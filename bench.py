@@ -25,6 +25,7 @@ One JSON line is printed (rank 0).  Its primary metric is the one that is define
             extrapolation to configs[2] stated.  Rank 0, --gpus 1 only.
 
 `--impl reference` times the same CPU restatements alone (TreeCorr itself is not installable here).
+`--dump-outputs DIR` saves the bin sums of the last timed pair count (DIR/npairs.npy, sumw.npy, sumwkk.npy).
 """
 import argparse
 import json
@@ -57,7 +58,14 @@ def parse_args():
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--skip-other", action="store_true", help="skip the cfg2 / cfg4b / cfg5 side measurements")
     ap.add_argument("--cpu-rows", type=int, default=20000, help="rows of the pair matrix in the CPU sample")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the bin sums of the last timed 2PCF step as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -385,6 +393,8 @@ def run_ours(args):
     res, step_ms, kern_ms = timed_counts(mx, edges, args.steps)
     launches += 2 * args.steps  # pairbin_boxes_kernel + pairbin_kernel (ours); the counter memset and torch fills are not counted
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_pairbin(args.dump_outputs, res.cpu().numpy(), counts_are_words)
     counted = total_count(res)
     total_ms = float(np.sum(step_ms))
     value = npairs_total * args.steps / (total_ms * 1e-3)
@@ -532,6 +542,17 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
     if world > 1:
         tdist.destroy_process_group()
+
+
+def dump_pairbin(out_dir, host, counts_are_words):
+    """What backend.pairbin returns for the last timed step -- pair counts, sum w and sum w k k, each shaped
+    (catalogues, NBINS * NBINS) -- as float64 .npy files.  The inputs are seeded, so two builds run with the same
+    arguments can be compared output for output: the counts and sum w exactly, sum w k k to rounding (the kernel
+    accumulates it with FP64 atomics, whose order varies from run to run)."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = np.ascontiguousarray(host[0]).view(np.int64) if counts_are_words else host[0]
+    for name, a in (("npairs", counts), ("sumw", host[1]), ("sumwkk", host[2])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def _ev(torch, fn, reps=2):

@@ -1,9 +1,8 @@
 """TEST INFRASTRUCTURE: a CPU stand-in for treegp_b200.backend built on the oracle.
 
-Used only by tests/test_reference_suite.py to run the REFERENCE's own test files (unchanged) against the
-host mirror in a container without a GPU: it checks the drop-in API (names, signatures, attributes, optimiser
-plumbing, MIGRAD stand-in, meanify, E/B utilities), not the CUDA arithmetic -- that is what the `-m gpu`
-parity tests are for.  The product never imports this module.
+Used only by tests/golden_r2_checks.py to run the host logic around the device operators (optimiser loops,
+bootstrap bookkeeping, E/B utilities) on a machine without a GPU; it does not check the CUDA arithmetic -- that
+is what the `-m gpu` parity tests are for.  The product never imports this module.
 """
 import numpy as np
 import scipy.linalg as sla
