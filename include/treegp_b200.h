@@ -138,6 +138,26 @@ int tgp_loglike_env(const double* X, const double* y, const double* yerr2, int64
                     const tgp_kernel* k /*host*/, double* work, int64_t ld, double* alpha, int want_alpha,
                     double* out, int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, void* stream);
 
+/* ---- (2c) selected inverse and the analytic log-likelihood gradient ----------------------------------------------
+ * The reference fits by L-BFGS-B with a forward-difference gradient (log_likelihood.py:56-57: n_theta + 1
+ * factorisations per step); these entries give the exact gradient for about three factorisations' worth of work.
+ * scratch: 16-byte aligned device buffer of tgp_selinv_work_doubles(N) doubles. */
+int64_t tgp_selinv_work_doubles(int64_t N);
+
+/* In place on a factor L from tgp_potrf / tgp_potrf_env / tgp_loglike[_env] (row-major, ld even >= N): Z = (L L^T)^-1
+ * on every entry of the envelope row_end (HOST, as tgp_potrf_env; NULL = dense), written to the lower triangle and
+ * mirrored into the upper one.  Entries outside the envelope are neither read nor written. */
+int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_end /*host*/, int64_t nblocks, double* scratch,
+               void* stream);
+
+/* tgp_loglike[_env] with want_alpha (alpha = K^-1 y), then tgp_selinv on the factor in `work`, then one contraction:
+ * out: device double[7] = {logL, chi2, logdet, d logL / d ln amp, d logL / d m00, d logL / d m01, d logL / d m11}
+ * (1-D: the last two are 0).  On exit `work` holds Z inside the envelope.  When *info != 0, out[0] = -inf and the
+ * gradient is 0.  Repeated calls give bit-identical results. */
+int tgp_loglike_grad(const double* X, const double* y, const double* yerr2, int64_t N,
+                     const tgp_kernel* k /*host*/, double* work, int64_t ld, double* alpha, double* out,
+                     int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, double* scratch, void* stream);
+
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 
 /* mean[m] = sum_n K(Xs_m, X_n) alpha_n without materialising K(Xs, X).

@@ -47,6 +47,9 @@ SIGNATURES = {
     "tgp_potrf_env": [_vp, _i64, _i64, _vp, _i64, _i64, _vp, _vp],
     "tgp_trsm_rows_env": [_vp, _i64, _i64, _vp, _i64, _vp, _i64, _i64, _vp],
     "tgp_loglike_env": [_vp, _vp, _vp, _i64, _kp, _vp, _i64, _vp, ctypes.c_int, _vp, _vp, _vp, _i64, _vp],
+    "tgp_selinv_work_doubles": [_i64],
+    "tgp_selinv": [_vp, _i64, _i64, _vp, _i64, _vp, _vp],
+    "tgp_loglike_grad": [_vp, _vp, _vp, _i64, _kp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -78,6 +81,7 @@ SIGNATURES = {
     "tgp_microbench_fp64": [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)],
 }
 _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctypes.c_int64,
+             "tgp_selinv_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 

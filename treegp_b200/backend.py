@@ -224,6 +224,53 @@ def loglike(X, y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
     return out, info, alpha, work
 
 
+def _selinv_scratch(N, device):
+    return torch.empty(int(_cabi.load().tgp_selinv_work_doubles(int(N))), dtype=F64, device=device)
+
+
+def selinv(L, N, row_end=None):
+    """In place on the factor L (workspace of potrf / loglike): Z = (L L^T)^-1 on every entry of the envelope row_end
+    (None: the whole matrix), lower triangle mirrored into the upper one (tgp_selinv).  Returns L."""
+    scratch = _selinv_scratch(N, L.device)
+    re = None if row_end is None else _host_i64(row_end)
+    check(_cabi.load().tgp_selinv(_p(L), int(N), L.stride(0), re, 0 if row_end is None else len(row_end), _p(scratch),
+                                  _stream()), "tgp_selinv")
+    return L
+
+
+def selinv_flops(row_end, n):
+    """Flop count of tgp_selinv for that envelope (None: dense): per block column of width w with m envelope rows
+    below it, w^3 (the inverse of the diagonal block) + 2 w^2 m (T) + 2 w m^2 (Z[R, J]) + w^3 + w^2 m (Z[J, J])."""
+    ob = envelope_block()
+    k = np.arange(0, n, ob, dtype=np.float64)
+    w = np.minimum(ob, n - k)
+    re = np.full(len(k), float(n)) if row_end is None else np.asarray(row_end, dtype=np.float64)
+    m = np.maximum.accumulate(np.clip(re, k + w, n)) - (k + w)
+    return float(np.sum(2.0 * w ** 3 + 3.0 * w * w * m + 2.0 * w * m * m))
+
+
+def loglike_grad(X, y, yerr2, kdesc, work=None, row_end=None):
+    """Log-likelihood and its gradient in one call (tgp_loglike_grad).  Returns (out[7] = logL, chi2, logdet,
+    d logL / d ln amp, d logL / d m00, d m01, d m11; info; alpha = K^-1 y; work, which holds Z = K^-1 inside the
+    envelope afterwards).  row_end as for loglike (X, y, yerr2 sorted along the envelope's axis)."""
+    X = as_points(X)
+    _check_dims(kdesc, X)
+    N = X.shape[0]
+    if work is None:
+        work = alloc_matrix(N + 1, N, X.device)
+    if work.shape[0] < N + 1:
+        raise ValueError("loglike_grad workspace needs N+1 rows")
+    alpha = torch.empty(N, dtype=F64, device=X.device)
+    out = torch.zeros(7, dtype=F64, device=X.device)
+    info = torch.zeros(1, dtype=torch.int32, device=X.device)
+    scratch = _selinv_scratch(N, X.device)
+    re = None if row_end is None else _host_i64(row_end)
+    check(_cabi.load().tgp_loglike_grad(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
+                                        _p(alpha), _p(out), _p(info), re, 0 if row_end is None else len(row_end),
+                                        _p(scratch), _stream()), "tgp_loglike_grad")
+    return out, info, alpha, work
+
+
 TRUNC_MIN_M, TRUNC_MIN_N = 16384, 2048   # below this the plain kernel is launch-bound anyway
 
 

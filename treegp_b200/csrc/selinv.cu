@@ -1,0 +1,328 @@
+// Selected inverse of the covariance inside the envelope of its Cholesky factor, and the analytic gradient of the
+// marginal log-likelihood that it makes possible.
+//
+// tgp_selinv: Z = (L L^T)^-1 on every entry of the envelope of L (the dense matrix when there is no envelope), by the
+// blocked Takahashi recurrence.  For the OB-wide block columns J from last to first, R = [end of J, row_end[J]) the
+// envelope rows below J, L11 = L[J, J], L21 = L[R, J]:
+//   W       = L11^-1                      (stored as -W^T: tgp_trsm_rows on -I, i.e. the DMMA halving solver)
+//   T^T     = W^T L21^T                   (gemm_nt_sub into zeroed scratch)
+//   Z[R, J] = -Z[R, R] T                  (gemm_nt_sub over L21's storage; Z[R, R] is dense in memory thanks to the
+//                                          mirror into the upper triangle, which the kernel build never writes)
+//   Z[J, J] = W^T W - T^T Z[R, J]         (two lower-only gemm_nt_sub, the second with B = the mirrored Z[J, R])
+// Z[R, R] lies inside the envelope because row_end is non-decreasing, so nothing outside it is read or written.
+// Flops: 2 w m^2 + 3 w^2 m + 2 w^3 per block column (w = OB, m = |R|), about twice the factorisation's w m^2 + w^2 m.
+//
+// tgp_loglike_grad: K build -> factorisation -> both sweeps (alpha = K^-1 y) -> tgp_selinv -> one fused contraction
+// over the lower triangle inside the envelope: with w_ij = alpha_i alpha_j - Z_ij and K_ij = a f(q_ij),
+//   d logL / d ln a = 1/2 sum_ij w_ij a f(q_ij),   d logL / d m_uv = 1/2 sum_ij w_ij a f'(q_ij) d q_ij / d m_uv.
+#include <string.h>
+#include <vector>
+#include "tgp_common.cuh"
+#include "profile_dq.cuh"
+
+extern "C" int tgp_trsm_rows(const double* L, int64_t N, int64_t ld, double* B, int64_t M, int64_t ldb, void* stream);
+extern "C" int tgp_gemm_nt_sub(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
+                               const double* B, int64_t ldb, int64_t Kd, int lower_only, void* stream);
+extern "C" int tgp_loglike(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
+                           double* work, int64_t ld, double* alpha, int want_alpha, double* out, int32_t* info,
+                           void* stream);
+extern "C" int tgp_loglike_env(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
+                               double* work, int64_t ld, double* alpha, int want_alpha, double* out, int32_t* info,
+                               const int64_t* row_end, int64_t nblocks, void* stream);
+extern "C" int tgp_envelope_block(void);
+
+constexpr int SB = 512;            // block columns of the recurrence: the envelope's block (tgp_envelope_block)
+constexpr int GT = 64;             // contraction tile edge
+constexpr int GT_THREADS = 256;
+
+static int64_t even64(int64_t n) { return (n + 1) & ~(int64_t)1; }
+static int64_t grad_tiles(int64_t N) {
+  const int64_t nt = tgp_cdiv(N, GT);
+  return nt * (nt + 1) / 2;
+}
+
+extern "C" int64_t tgp_selinv_work_doubles(int64_t N) {
+  if (N < 1) N = 1;
+  const int64_t selinv = 2 * (int64_t)SB * SB + (int64_t)SB * even64(N);   // -W^T, W^T, T^T
+  const int64_t partials = 4 * grad_tiles(N);                               // contraction partial sums
+  return (selinv > partials ? selinv : partials) + even64(tgp_cdiv(N, SB));  // + the device copy of row_end
+}
+
+// ---- small helpers --------------------------------------------------------------------------------------------
+// S (n x n, pitch lds) = -I
+__global__ void neg_identity_kernel(double* __restrict__ S, int n, int64_t lds) {
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < (int64_t)n * n;
+       idx += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = idx / n, c = idx % n;
+    S[r * lds + c] = (r == c) ? -1.0 : 0.0;
+  }
+}
+
+// D (n x n) = -S
+__global__ void negate_kernel(const double* __restrict__ S, double* __restrict__ D, int n, int64_t ld) {
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < (int64_t)n * n;
+       idx += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = idx / n, c = idx % n;
+    D[r * ld + c] = -S[r * ld + c];
+  }
+}
+
+// dst[c][r] = src[r][c] for the rows x cols block src (both with pitch ld).  lower_only: src == dst is a square
+// diagonal block whose strict lower triangle is mirrored into its upper triangle (disjoint entries: no race).
+__global__ void __launch_bounds__(256)
+mirror_kernel(const double* __restrict__ src, double* __restrict__ dst, int64_t rows, int64_t cols, int64_t ld,
+              int lower_only) {
+  __shared__ double t[32][33];
+  const int64_t r0 = (int64_t)blockIdx.y * 32, c0 = (int64_t)blockIdx.x * 32;
+  if (lower_only && c0 > r0) return;
+  const int tx = threadIdx.x, ty = threadIdx.y;   // 32 x 8
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t r = r0 + ty + 8 * i, c = c0 + tx;
+    if (r < rows && c < cols && (!lower_only || c < r)) t[ty + 8 * i][tx] = src[r * ld + c];
+  }
+  __syncthreads();
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t c = c0 + ty + 8 * i, r = r0 + tx;   // write row c of dst, coalesced along r
+    if (r < rows && c < cols && (!lower_only || c < r)) dst[c * ld + r] = t[tx][ty + 8 * i];
+  }
+}
+
+static int mirror_launch(const double* src, double* dst, int64_t rows, int64_t cols, int64_t ld, int lower_only,
+                         cudaStream_t st) {
+  if (rows <= 0 || cols <= 0) return TGP_OK;
+  dim3 grid((unsigned)tgp_cdiv(cols, 32), (unsigned)tgp_cdiv(rows, 32));
+  TGP_CHECK_ARG(grid.y <= 65535u, "too many rows for one launch");
+  mirror_kernel<<<grid, dim3(32, 8), 0, st>>>(src, dst, rows, cols, ld, lower_only);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+static int check_args_mat(const double* A, int64_t N, int64_t ld) {
+  return N <= 0 || ld < N || !A || (ld & 1) || ((uintptr_t)A & 15);
+}
+static int check_env(const int64_t* row_end, int64_t nblocks, int64_t N) {
+  return row_end != nullptr && nblocks != tgp_cdiv(N, (int64_t)SB);
+}
+
+// Row ends as the factorisation uses them: clamped to [end of the block, N] and made non-decreasing.
+static std::vector<int64_t> clamped_row_end(const int64_t* row_end, int64_t N) {
+  const int64_t nb = tgp_cdiv(N, (int64_t)SB);
+  std::vector<int64_t> re((size_t)nb);
+  int64_t prev = 0;
+  for (int64_t b = 0; b < nb; ++b) {
+    const int64_t c1 = (b + 1) * SB < N ? (b + 1) * SB : N;
+    int64_t r = row_end ? row_end[b] : N;
+    if (r < prev) r = prev;
+    if (r < c1) r = c1;
+    if (r > N) r = N;
+    re[(size_t)b] = prev = r;
+  }
+  return re;
+}
+
+static int selinv_run(double* A, int64_t N, int64_t ld, const std::vector<int64_t>& re, double* scratch,
+                      cudaStream_t st) {
+  void* sv = (void*)st;
+  double* NWT = scratch;                  // -W^T, SB x SB
+  double* WT = scratch + SB * SB;         //  W^T, SB x SB
+  double* TT = scratch + 2 * SB * SB;     //  T^T, SB x ldt
+  const int64_t ldt = even64(N);
+  const unsigned eg = 2 * (unsigned)tgp_num_sms();
+  for (int64_t b = (int64_t)re.size() - 1; b >= 0; --b) {
+    const int64_t k = b * SB, w = (N - k < SB) ? (N - k) : SB, c1 = k + w, m = re[(size_t)b] - c1;
+    double* Akk = A + k * ld + k;
+    double* L21 = A + c1 * ld + k;        // becomes Z[R, J]
+    double* ZJR = A + k * ld + c1;        // upper-triangle storage of Z[J, R]
+    int rc;
+    neg_identity_kernel<<<eg, 256, 0, st>>>(NWT, (int)w, SB);
+    TGP_LAUNCH_CHECK();
+    rc = tgp_trsm_rows(Akk, w, ld, NWT, w, SB, sv);            // rows of -I times L11^-T: -W^T
+    if (rc) return rc;
+    negate_kernel<<<eg, 256, 0, st>>>(NWT, WT, (int)w, SB);
+    TGP_LAUNCH_CHECK();
+    if (m > 0) {
+      TGP_CUDA(cudaMemset2DAsync(TT, ldt * sizeof(double), 0, m * sizeof(double), w, st));
+      rc = tgp_gemm_nt_sub(TT, w, m, ldt, NWT, SB, L21, ld, w, 0, sv);              // T^T = W^T L21^T
+      if (rc) return rc;
+      TGP_CUDA(cudaMemset2DAsync(L21, ld * sizeof(double), 0, w * sizeof(double), m, st));
+      rc = tgp_gemm_nt_sub(L21, m, w, ld, A + c1 * ld + c1, ld, TT, ldt, m, 0, sv);  // Z[R, J] = -Z[R, R] T
+      if (rc) return rc;
+      rc = mirror_launch(L21, ZJR, m, w, ld, 0, st);
+      if (rc) return rc;
+    }
+    TGP_CUDA(cudaMemset2DAsync(Akk, ld * sizeof(double), 0, w * sizeof(double), w, st));
+    rc = tgp_gemm_nt_sub(Akk, w, w, ld, NWT, SB, WT, SB, w, 1, sv);                 // + W^T W
+    if (rc) return rc;
+    if (m > 0) {
+      rc = tgp_gemm_nt_sub(Akk, w, w, ld, TT, ldt, ZJR, ld, m, 1, sv);               // - T^T Z[R, J]
+      if (rc) return rc;
+    }
+    rc = mirror_launch(Akk, Akk, w, w, ld, 1, st);
+    if (rc) return rc;
+  }
+  return TGP_OK;
+}
+
+extern "C" int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_end, int64_t nblocks, double* scratch,
+                          void* stream) {
+  TGP_CHECK_ARG(!check_args_mat(L, N, ld), "L must be 16-byte aligned with even ld >= N > 0");
+  TGP_CHECK_ARG(!check_env(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(scratch && ((uintptr_t)scratch & 15) == 0,
+                "scratch: 16-byte aligned buffer of tgp_selinv_work_doubles(N) doubles");
+  return selinv_run(L, N, ld, clamped_row_end(row_end, N), scratch, (cudaStream_t)stream);
+}
+
+// ---- gradient contraction ---------------------------------------------------------------------------------------
+// One CTA per 64 x 64 tile (I >= J) of the lower triangle; tiles whose rows all lie below the envelope of their
+// block column write zeros.  Thread: 2 adjacent columns x 8 rows, as the K build (kmat.cu).  Partial sums
+// {sum w a f, sum w a f' dx^2, sum w a f' 2 dx dy, sum w a f' dy^2} (off-diagonal pairs twice) per tile; the finishing
+// kernel adds the tiles in index order, so the result does not depend on scheduling.
+//
+// Pairs outside the envelope are dropped, as by the factorisation: their q is at least tgp_profile_qcut, where
+// f <= 1e-40 and |f'(q) q| is below (qcut / 2) f(qcut) ~ 2e-38 (RBF, q f' = -q f / 2 at qcut = 185), below
+// 1e-36 for the von Karman profile (qcut = 224: |q f'| = pi sqrt(q) K_{1/6}/K_{5/6} f ~ 47 f) and below
+// sqrt(q)/2 f, sqrt(3q) f, 5/6 (1 + sqrt(5q)) sqrt(5q) f ~ 1e-37 for the Matern families -- every dropped term is
+// below 1e-36 a |w_ij| |dq / dm| / q.
+template <int FAM>
+__global__ void __launch_bounds__(GT_THREADS)
+grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double* __restrict__ Z, int64_t ld,
+                     const double* __restrict__ alpha, const int64_t* __restrict__ re_dev,
+                     double* __restrict__ partials, const double* __restrict__ phi_g) {
+  __shared__ double xr[GT], yr[GT], ar[GT], xc[GT], yc[GT], ac[GT];
+  __shared__ double red[GT_THREADS / 32][4];
+  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  const int64_t t = blockIdx.x;
+  int64_t I = (int64_t)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
+  while (I * (I + 1) / 2 > t) --I;
+  while ((I + 1) * (I + 2) / 2 <= t) ++I;
+  const int64_t J = t - I * (I + 1) / 2;
+  const int64_t r0 = I * GT, c0 = J * GT;
+  const int64_t rend = re_dev ? re_dev[c0 / SB] : N;   // one past the last envelope row of this block column
+  const int tid = threadIdx.x;
+  if (r0 >= rend) {
+    if (tid < 4) partials[4 * t + tid] = 0.0;
+    return;
+  }
+  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (tid < GT) {
+    const int64_t r = r0 + tid;
+    const bool ok = r < N;
+    xr[tid] = ok ? X[r * kd.ndim] : 0.0;
+    yr[tid] = (ok && kd.ndim == 2) ? X[r * 2 + 1] : 0.0;
+    ar[tid] = ok ? alpha[r] : 0.0;
+  } else if (tid < 2 * GT) {
+    const int l = tid - GT;
+    const int64_t c = c0 + l;
+    const bool ok = c < N;
+    xc[l] = ok ? X[c * kd.ndim] : 0.0;
+    yc[l] = (ok && kd.ndim == 2) ? X[c * 2 + 1] : 0.0;
+    ac[l] = ok ? alpha[c] : 0.0;
+  }
+  __syncthreads();
+  const int lane = tid & 31, warp = tid >> 5;
+  double s[4] = {0.0, 0.0, 0.0, 0.0};
+#pragma unroll(FAM == TGP_FAM_VONKARMAN ? 1 : GT / 8)
+  for (int rr = 0; rr < GT / 8; ++rr) {
+    const int rl = warp + 8 * rr;
+    const int64_t rg = r0 + rl;
+    if (rg >= N || rg >= rend) continue;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int cl = 2 * lane + h;
+      const int64_t cg = c0 + cl;
+      if (cg > rg) continue;
+      const double dx = xr[rl] - xc[cl], dy = yr[rl] - yc[cl];
+      const double q = tgp_qform(kd, dx, dy);
+      const double wij = (rg == cg ? 1.0 : 2.0) * (ar[rl] * ac[cl] - Z[rg * ld + cg]);
+      double f = tgp_profile<FAM>(q, phi_s);
+      // K(X, X) of the von Karman kernels is 0 between distinct coincident points (kmat.cu, kernels.py:253-262)
+      if (FAM == TGP_FAM_VONKARMAN && q == 0.0 && rg != cg) f = 0.0;
+      s[0] = fma(wij, kd.amp * f, s[0]);
+      if (q > 0.0) {
+        const double d = wij * kd.amp * tgp_profile_dq<FAM>(q, phi_s);
+        s[1] = fma(d, dx * dx, s[1]);
+        s[2] = fma(d, 2.0 * dx * dy, s[2]);
+        s[3] = fma(d, dy * dy, s[3]);
+      }
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s[c] += __shfl_xor_sync(0xffffffffu, s[c], o);
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int c = 0; c < 4; ++c) red[warp][c] = s[c];
+  }
+  __syncthreads();
+  if (tid < 4) {
+    double v = 0.0;
+    for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi][tid];
+    partials[4 * t + tid] = v;
+  }
+}
+
+// out[3..6] = 1/2 the tile sums in tile order; 0 when the factorisation failed (out[0] is then -inf already).
+__global__ void __launch_bounds__(1024)
+grad_finish_kernel(const double* __restrict__ partials, int64_t ntiles, const int32_t* __restrict__ info,
+                   double* __restrict__ out) {
+  __shared__ double red[32][4];
+  double s[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int64_t t = threadIdx.x; t < ntiles; t += blockDim.x) {
+#pragma unroll
+    for (int c = 0; c < 4; ++c) s[c] += partials[4 * t + c];
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int c = 0; c < 4; ++c) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s[c] += __shfl_xor_sync(0xffffffffu, s[c], o);
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int c = 0; c < 4; ++c) red[warp][c] = s[c];
+  }
+  __syncthreads();
+  if (threadIdx.x < 4) {
+    double v = 0.0;
+    for (int wi = 0; wi < 32; ++wi) v += red[wi][threadIdx.x];
+    out[3 + threadIdx.x] = (*info != 0) ? 0.0 : 0.5 * v;
+  }
+}
+
+extern "C" int tgp_loglike_grad(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
+                                double* work, int64_t ld, double* alpha, double* out, int32_t* info,
+                                const int64_t* row_end, int64_t nblocks, double* scratch, void* stream) {
+  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+  TGP_CHECK_ARG(N > 0 && X && y && alpha && out && info, "null pointer / N");
+  TGP_CHECK_ARG(!check_args_mat(work, N, ld), "work must be 16-byte aligned with even ld >= N");
+  TGP_CHECK_ARG(!check_env(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(scratch && ((uintptr_t)scratch & 15) == 0,
+                "scratch: 16-byte aligned buffer of tgp_selinv_work_doubles(N) doubles");
+  const int64_t ntiles = grad_tiles(N);
+  TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
+  cudaStream_t st = (cudaStream_t)stream;
+  int rc = row_end ? tgp_loglike_env(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream)
+                   : tgp_loglike(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, stream);
+  if (rc) return rc;
+  const std::vector<int64_t> re = clamped_row_end(row_end, N);
+  rc = selinv_run(work, N, ld, re, scratch, st);
+  if (rc) return rc;
+  // the selected-inverse scratch is free again: tile partials at the front, the envelope at the back
+  int64_t* re_dev = nullptr;
+  if (row_end) {
+    re_dev = reinterpret_cast<int64_t*>(scratch + tgp_selinv_work_doubles(N) - even64((int64_t)re.size()));
+    TGP_CUDA(cudaMemcpyAsync(re_dev, re.data(), re.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  }
+  const KDesc kd = make_kdesc(k);
+  const double* phi = tgp_phi_device();
+  TGP_FAMILY_SWITCH(k->family, (grad_contract_kernel<FAM><<<(unsigned)ntiles, GT_THREADS, 0, st>>>(
+                                   X, N, kd, work, ld, alpha, re_dev, scratch, phi)));
+  TGP_LAUNCH_CHECK();
+  grad_finish_kernel<<<1, 1024, 0, st>>>(scratch, ntiles, info, out);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}

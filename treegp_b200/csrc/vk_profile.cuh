@@ -104,3 +104,61 @@ TGP_HD double tgp_vk_profile(double q, const double* __restrict__ phi) {
   // fmax guards the one-ulp case where u >= 1/4 but 2 pi sqrt(q) rounds just below 1
   return tgp_vk_large(fmax(TGP_2PI * sqrt(q), 1.0), phi);
 }
+
+// df/dq = -2 pi^2 2^(1/6)/Gamma(5/6) z^(-1/6) K_{1/6}(z), z = 2 pi sqrt(q), from the same series and tables as f:
+//   u < 1/4 : f = A(u) - u^(5/6) B(u)  ->  df/dq = pi^2 [A'(u) - u^(5/6) (5/6 B(u) / u + B'(u))]
+//   z >= 1  : f = C e^-z psi(z), psi a polynomial in s = 2 m - 3 (m the mantissa of z, ds/dz = 2 / 2^e)
+//             ->  df/dz = C e^-z (psi' - psi),  df/dq = df/dz 2 pi^2 / z.
+// Singular (-inf) at q = 0: the caller gives coincident points no metric derivative.
+TGP_HD double tgp_vk_profile_dq(double q, const double* __restrict__ phi) {
+  const double u = TGP_PI2 * q;
+  if (u < 0.25) {
+#define TGP_A_TERM(k, c) const double a##k = c;
+#define TGP_B_TERM(k, c) const double b##k = c;
+    TGP_VK_SER_A(TGP_A_TERM)
+    TGP_VK_SER_B(TGP_B_TERM)
+#undef TGP_A_TERM
+#undef TGP_B_TERM
+    double b = b10, da = 10.0 * a10, db = 10.0 * b10;
+    b = tgp_fma(b, u, b9);  da = tgp_fma(da, u, 9.0 * a9);  db = tgp_fma(db, u, 9.0 * b9);
+    b = tgp_fma(b, u, b8);  da = tgp_fma(da, u, 8.0 * a8);  db = tgp_fma(db, u, 8.0 * b8);
+    b = tgp_fma(b, u, b7);  da = tgp_fma(da, u, 7.0 * a7);  db = tgp_fma(db, u, 7.0 * b7);
+    b = tgp_fma(b, u, b6);  da = tgp_fma(da, u, 6.0 * a6);  db = tgp_fma(db, u, 6.0 * b6);
+    b = tgp_fma(b, u, b5);  da = tgp_fma(da, u, 5.0 * a5);  db = tgp_fma(db, u, 5.0 * b5);
+    b = tgp_fma(b, u, b4);  da = tgp_fma(da, u, 4.0 * a4);  db = tgp_fma(db, u, 4.0 * b4);
+    b = tgp_fma(b, u, b3);  da = tgp_fma(da, u, 3.0 * a3);  db = tgp_fma(db, u, 3.0 * b3);
+    b = tgp_fma(b, u, b2);  da = tgp_fma(da, u, 2.0 * a2);  db = tgp_fma(db, u, 2.0 * b2);
+    b = tgp_fma(b, u, b1);  da = tgp_fma(da, u, a1);        db = tgp_fma(db, u, b1);
+    b = tgp_fma(b, u, b0);
+    (void)a0;
+    const double p = sqrt(u) * cbrt(u);   // u^(5/6)
+    return TGP_PI2 * tgp_fma(-p, (5.0 / 6.0) * b / u + db, da);
+  }
+  const double z = fmax(TGP_2PI * sqrt(q), 1.0);
+  if (z > 746.0) return 0.0;
+  uint64_t bits;
+#if defined(__CUDA_ARCH__)
+  bits = (uint64_t)__double_as_longlong(z);
+#else
+  memcpy(&bits, &z, sizeof bits);
+#endif
+  const int e = (int)(bits >> 52) - 1023;
+  uint64_t mb = (bits & 0x000FFFFFFFFFFFFFull) | 0x3FF0000000000000ull;
+  double m;
+#if defined(__CUDA_ARCH__)
+  m = __longlong_as_double((long long)mb);
+#else
+  memcpy(&m, &mb, sizeof m);
+#endif
+  const double s = tgp_fma(2.0, m, -3.0);
+  const double* c = phi + (e - TGP_VK_E_MIN) * TGP_VK_PHI_STRIDE;
+  double psi = c[TGP_VK_PHI_STRIDE - 1], dpsi = (TGP_VK_PHI_STRIDE - 1) * c[TGP_VK_PHI_STRIDE - 1];
+#pragma unroll
+  for (int k = TGP_VK_PHI_STRIDE - 2; k >= 1; --k) {
+    psi = tgp_fma(psi, s, c[k]);
+    dpsi = tgp_fma(dpsi, s, k * c[k]);
+  }
+  psi = tgp_fma(psi, s, c[0]);
+  const double dpsi_dz = dpsi * ldexp(2.0, -e);
+  return TGP_VK_C_INF * exp(-z) * (dpsi_dz - psi) * (2.0 * TGP_PI2 / z);
+}

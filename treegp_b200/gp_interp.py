@@ -188,6 +188,40 @@ class GPInterpolation(object):
             a[env["order"]] = alpha
             self._alpha = a.cpu().numpy()
 
+    def loo_predict(self):
+        """Extension (not in the reference): leave-one-out predictions at every training point, in the caller's
+        order, without refitting -- (mean, var) with mean_i = y_i - alpha_i / Z_ii and var_i = 1 / Z_ii - y_err_i^2,
+        Z = (K + diag(y_err^2))^-1 (its diagonal from the selected inverse, tgp_selinv), y_err after the white noise.
+        This is what predict / predict_var return at X_i from the other N - 1 points with the same kernel; the
+        normalising mean and the mean function keep their all-point values and are added back as predict does.
+        Factorises into a workspace of its own: the cached factor of predict_var / return_cov stays as it is."""
+        y = np.asarray(self._y - self._mean - self._spatial_average, dtype=np.float64).reshape(-1)
+        Xd = backend.as_points(self._X)
+        n = Xd.shape[0]
+        desc = lower_kernel(self.kernel, Xd.shape[1])
+        e2_host = np.asarray(self._y_err, dtype=np.float64).reshape(-1) ** 2
+        e2, yd = backend.to_device(e2_host), backend.to_device(y)
+        env = backend.plan_envelope(Xd, desc) if self.BANDED_SOLVE else None
+        if env is not None:
+            Xd, yd, e2 = Xd[env["order"]].contiguous(), yd[env["order"]].contiguous(), e2[env["order"]].contiguous()
+        row_end = None if env is None else env["row_end"]
+        _, info, alpha, ws = backend.loglike(Xd, yd, e2, desc, want_alpha=True, row_end=row_end)
+        bad = int(info.item())
+        if bad < 0:
+            raise _cabi.TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % bad)
+        if bad != 0:
+            raise np.linalg.LinAlgError("%d-th leading minor of the array is not positive definite" % bad)
+        backend.selinv(ws, n, row_end=row_end)
+        zdiag = ws[:, :n].diagonal()
+        if env is not None:
+            order = env["order"]
+            a, z = alpha.new_empty(alpha.shape), zdiag.new_empty(zdiag.shape)
+            a[order], z[order] = alpha, zdiag
+            alpha, zdiag = a, z
+        alpha, zdiag = alpha.cpu().numpy(), zdiag.cpu().numpy()
+        mean = y - alpha / zdiag + self._mean + self._spatial_average
+        return mean, 1.0 / zdiag - e2_host
+
     def return_gp_predict(self, y, X1, X2, kernel, y_err, return_cov=False):
         """GP algebra for residuals y at X1 with errors y_err, evaluated at X2 with `kernel`
         (gp_interp.py:168-194): returns (mean, covariance-or-None)."""

@@ -27,7 +27,8 @@ from sklearn.gaussian_process.kernels import (
 from . import _cabi
 from ._cabi import TgpKernel
 
-__all__ = ["eval_kernel", "AnisotropicRBF", "VonKarman", "AnisotropicVonKarman", "lower_kernel"]
+__all__ = ["eval_kernel", "AnisotropicRBF", "VonKarman", "AnisotropicVonKarman", "lower_kernel",
+           "lower_kernel_jacobian"]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -315,3 +316,65 @@ def lower_kernel(kernel, ndim):
     if isinstance(base, RBF):
         return _descriptor(_cabi.FAM_RBF, ndim, amp, _iso_metric(base.length_scale, ndim, "RBF"))
     raise _cabi.TgpError("unsupported kernel for the B200 backend: %r" % (kernel,))
+
+
+def _metric_columns(dM, ndim):
+    """Symmetric 2 x 2 (or 1 x 1) derivative of the inverse metric -> rows (m00, m01, m11) of the Jacobian."""
+    dM = np.atleast_2d(dM)
+    if ndim == 1:
+        return np.array([dM[0, 0], 0.0, 0.0])
+    return np.array([dM[0, 0], dM[0, 1], dM[1, 1]])
+
+
+def _factor_jacobian(k, ndim):
+    """Columns d(ln a, m00, m01, m11) / d theta_k of one factor of the product, in the order of k.theta."""
+    if isinstance(k, ConstantKernel):
+        return [] if k.hyperparameter_constant_value.fixed else [np.array([1.0, 0.0, 0.0, 0.0])]
+    if isinstance(k, _MetricKernel):
+        if k.ndim != ndim:
+            raise ValueError("kernel is %d-D but coordinates are %d-D" % (k.ndim, ndim))
+        n, L = k.ndim, k._L
+        cols = []
+        for a in range(n):                                  # theta[a] = ln L[a, a]
+            dL = np.zeros((n, n))
+            dL[a, a] = L[a, a]
+            cols.append(dL)
+        for i, j in zip(*k._t):                             # theta[n + ...] = L[i, j], i > j
+            dL = np.zeros((n, n))
+            dL[i, j] = 1.0
+            cols.append(dL)
+        return [np.concatenate([[0.0], _metric_columns(dL @ L.T + L @ dL.T, ndim)]) for dL in cols]
+    if isinstance(k, (VonKarman, RBF)):   # Matern subclasses RBF; its nu is not a hyper-parameter
+        if k.hyperparameter_length_scale.fixed:
+            return []
+        ls = np.ravel(np.asarray(k.length_scale, dtype=float))
+        if ls.size == 1:   # one theta: d M / d ln l = -2 l^-2 I
+            return [np.concatenate([[0.0], _metric_columns(-2.0 * np.eye(ndim) / ls[0] ** 2, ndim)])]
+        if ls.size != ndim:
+            raise ValueError("length_scale has %d entries for %d-D coordinates" % (ls.size, ndim))
+        cols = []
+        for a in range(ndim):   # d M / d ln l_a = -2 l_a^-2 e_a e_a^T
+            dM = np.zeros((ndim, ndim))
+            dM[a, a] = -2.0 / ls[a] ** 2
+            cols.append(np.concatenate([[0.0], _metric_columns(dM, ndim)]))
+        return cols
+    raise _cabi.TgpError("unsupported kernel for the B200 backend: %r" % (k,))
+
+
+def lower_kernel_jacobian(kernel, ndim):
+    """(``lower_kernel(kernel, ndim)``, J): J is the 4 x n_theta Jacobian of (ln amp, m00, m01, m11) with respect to
+    ``kernel.theta`` -- columns in scikit-learn's theta order (a Product lists k1's then k2's), fixed
+    hyper-parameters absent.  The chain rule that turns tgp_loglike_grad's derivatives into d logL / d theta
+    (d logL / d theta = J^T g).  Accepts exactly what lower_kernel accepts."""
+    desc = lower_kernel(kernel, ndim)
+
+    def walk(k):
+        if isinstance(k, Product):
+            return walk(k.k1) + walk(k.k2)
+        return _factor_jacobian(k, ndim)
+
+    cols = walk(kernel)
+    J = np.stack(cols, axis=1) if cols else np.zeros((4, 0))
+    if J.shape[1] != len(kernel.theta):
+        raise _cabi.TgpError("unsupported kernel for the B200 backend (theta layout): %r" % (kernel,))
+    return desc, J

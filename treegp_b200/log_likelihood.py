@@ -12,7 +12,7 @@ import numpy as np
 from scipy import optimize
 
 from . import backend
-from .kernels import lower_kernel
+from .kernels import lower_kernel, lower_kernel_jacobian
 
 # Multi-GPU (SURVEY.md section 8e): the (n_theta + 1) likelihood evaluations of one forward-difference gradient
 # are independent.  With DISTRIBUTED_FD = True (or env TREEGP_B200_DIST_FD=1) and an initialised process group,
@@ -89,6 +89,31 @@ class log_likelihood(object):
             raise TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % int(info.item()))
         return value
 
+    # optimizer(): L-BFGS-B with the analytic gradient of log_likelihood_and_gradient (jac=True) instead of scipy's
+    # forward differences (n_theta + 1 evaluations per gradient, each component with ~1e-8 relative noise of logL)
+    ANALYTIC_GRADIENT = False
+
+    def log_likelihood_and_gradient(self, kernel):
+        """(log p(y | X, kernel), d log p / d kernel.theta) from one device call (tgp_loglike_grad: the factorisation,
+        the selected inverse Z = K^-1 inside its envelope and one contraction with alpha alpha^T - Z).  Same envelope
+        choice and -inf rule as log_likelihood; the gradient is 0 where the value is -inf."""
+        Xd, yd, e2, work = self._device_state()
+        desc, J = lower_kernel_jacobian(kernel, Xd.shape[1])
+        if not np.all(np.isfinite([desc.amp, desc.m00, desc.m01, desc.m11])):
+            return -np.inf, np.zeros(J.shape[1])
+        banded = self._envelope_inputs(desc)
+        if banded is None:
+            out, info, _, _ = backend.loglike_grad(Xd, yd, e2, desc, work=work)
+        else:
+            out, info, _, _ = backend.loglike_grad(banded[0], banded[1], banded[2], desc, work=work, row_end=banded[3])
+            self.n_banded_evaluations = getattr(self, "n_banded_evaluations", 0) + 1
+        self.n_evaluations += 1
+        o = out.cpu().numpy()
+        if o[0] != o[0]:
+            from ._cabi import TgpError
+            raise TgpError("tgp_loglike_grad: internal synchronisation timed out (info = %d)" % int(info.item()))
+        return float(o[0]), J.T @ o[3:7]
+
     @staticmethod
     def _value_and_fd_gradient(fun, rank, world):
         """f(theta) and its forward-difference gradient with the n_theta + 1 probes dealt round-robin to the
@@ -117,7 +142,8 @@ class log_likelihood(object):
 
     def optimizer(self, kernel):
         """Maximise the likelihood over theta starting from `kernel.theta` (scipy L-BFGS-B, no bounds,
-        forward-difference gradient) and return the fitted kernel; keeps `_kernel` and `_logL`."""
+        forward-difference gradient, or the analytic one when ANALYTIC_GRADIENT is set) and return the fitted kernel;
+        keeps `_kernel` and `_logL`."""
 
         def minus_logl(theta):
             return -self.log_likelihood(kernel.clone_with_theta(theta))
@@ -126,7 +152,13 @@ class log_likelihood(object):
         from . import dist
 
         rank, world = dist.rank_world(None)
-        if world > 1 and (DISTRIBUTED_FD or os.environ.get("TREEGP_B200_DIST_FD") == "1"):
+        if self.ANALYTIC_GRADIENT:
+            def minus_logl_and_grad(theta):
+                v, g = self.log_likelihood_and_gradient(kernel.clone_with_theta(theta))
+                return -v, -g
+
+            best = optimize.minimize(minus_logl_and_grad, kernel.theta, method="L-BFGS-B", jac=True)["x"]
+        elif world > 1 and (DISTRIBUTED_FD or os.environ.get("TREEGP_B200_DIST_FD") == "1"):
             best = optimize.minimize(self._value_and_fd_gradient(minus_logl, rank, world), kernel.theta,
                                      method="L-BFGS-B", jac=True)["x"]
         else:
