@@ -53,6 +53,18 @@ typedef struct {
   double m00, m01, m11; /* symmetric inverse metric; ndim==1 uses m00 only */
 } tgp_kernel;
 
+/* POD lowering of a Sum of such terms plus a WhiteKernel level (sklearn `c1 * A + c2 * B + WhiteKernel(w)`):
+ * K(X, X)_ij = sum_c amp_c f_c(q_c) + white [i == j];  K(Xs, X) = sum_c amp_c f_c(q_c) (sklearn's WhiteKernel(X, Y)
+ * is zero whenever Y is passed).  The von Karman rule of K(X, X) (0 between distinct coincident points) applies per
+ * term.  Only term[0 .. nterms-1] is read. */
+#define TGP_MAX_TERMS 4
+typedef struct {
+  int32_t nterms;               /* 1 .. TGP_MAX_TERMS stationary terms */
+  int32_t ndim;                 /* 1 or 2; every term's ndim must equal it */
+  double white;                 /* WhiteKernel level: diagonal of K(X, X) only; >= 0, 0 if absent */
+  tgp_kernel term[TGP_MAX_TERMS];
+} tgp_kernel_sum;
+
 int tgp_abi_version(void);
 const char* tgp_last_error(void);
 
@@ -157,6 +169,39 @@ int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_end /*host*/
 int tgp_loglike_grad(const double* X, const double* y, const double* yerr2, int64_t N,
                      const tgp_kernel* k /*host*/, double* work, int64_t ld, double* alpha, double* out,
                      int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, double* scratch, void* stream);
+
+/* ---- (2d) sum kernels: the entries above for a tgp_kernel_sum ---------------------------------------------------
+ * Same arguments, conventions and results as their single-term twins, with K built from every term and the white
+ * level.  A one-term sum with white == 0 runs the single-term kernels (K(Xs, X) and the means: any one-term sum), so
+ * it gives bit for bit what the single-term entry gives. */
+int tgp_kmat_sym_sum(const double* X, int64_t N, const tgp_kernel_sum* k /*host*/, const double* diag_add,
+                     double* out, int64_t ld, int lower_only, void* stream);
+int tgp_kmat_cross_sum(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k /*host*/,
+                       double* out, int64_t ld, void* stream);
+/* tgp_loglike (row_end == NULL) or tgp_loglike_env (row_end != NULL). */
+int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel_sum* k /*host*/,
+                    double* work, int64_t ld, double* alpha, int want_alpha, double* out, int32_t* info,
+                    const int64_t* row_end /*host*/, int64_t nblocks, void* stream);
+/* tgp_loglike_grad for a sum: out: device double[4 + 4 nterms] = {logL, chi2, logdet, then per term c
+ * d logL / d (ln amp_c, m00_c, m01_c, m11_c) at out[3 + 4c ..], then d logL / d ln white at out[3 + 4 nterms]
+ * (0 when white == 0)}.  scratch: 16-byte aligned, tgp_loglike_grad_sum_work_doubles(N, nterms) doubles. */
+int64_t tgp_loglike_grad_sum_work_doubles(int64_t N, int32_t nterms);
+int tgp_loglike_grad_sum(const double* X, const double* y, const double* yerr2, int64_t N,
+                         const tgp_kernel_sum* k /*host*/, double* work, int64_t ld, double* alpha, double* out,
+                         int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, double* scratch,
+                         void* stream);
+/* tgp_predict_mean / tgp_predict_mean_trunc for a sum (no white term: it is zero between distinct point sets).
+ * The truncated form skips a group only beyond every term's cut-off; the error bound is
+ * 1e-40 * sum_c |amp_c| * sum_n |alpha_n|. */
+int tgp_predict_mean_sum(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k /*host*/,
+                         const double* alpha, double* mean, void* stream);
+int tgp_predict_mean_trunc_sum(const double* Xs, int64_t M, const double* X, int64_t N,
+                               const tgp_kernel_sum* k /*host*/, const double* alpha, double* mean, double* work,
+                               void* stream);
+/* var[m] = sum_c amp_c + white - || L^-1 K(X, Xs_m) ||^2 (tgp_predict_var; row_end optional as tgp_predict_var_env). */
+int tgp_predict_var_sum(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k /*host*/,
+                        const double* L, int64_t ld, const int64_t* row_end /*host*/, int64_t nblocks, double* work,
+                        int64_t chunk, double* var, void* stream);
 
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 

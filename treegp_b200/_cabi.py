@@ -23,12 +23,22 @@ class TgpKernel(ctypes.Structure):
                 ("m00", ctypes.c_double), ("m01", ctypes.c_double), ("m11", ctypes.c_double)]
 
 
+MAX_TERMS = 4   # TGP_MAX_TERMS
+
+
+class TgpKernelSum(ctypes.Structure):
+    """POD sum descriptor `tgp_kernel_sum`: nterms stationary terms plus a WhiteKernel level."""
+    _fields_ = [("nterms", ctypes.c_int32), ("ndim", ctypes.c_int32), ("white", ctypes.c_double),
+                ("term", TgpKernel * MAX_TERMS)]
+
+
 class TgpError(RuntimeError):
     pass
 
 
 _vp, _i64, _i32, _f64 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32, ctypes.c_double
 _kp = ctypes.POINTER(TgpKernel)
+_ksp = ctypes.POINTER(TgpKernelSum)
 
 # name -> argtypes; every entry returns int (tgp_status) unless listed in _RESTYPES
 SIGNATURES = {
@@ -50,6 +60,14 @@ SIGNATURES = {
     "tgp_selinv_work_doubles": [_i64],
     "tgp_selinv": [_vp, _i64, _i64, _vp, _i64, _vp, _vp],
     "tgp_loglike_grad": [_vp, _vp, _vp, _i64, _kp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
+    "tgp_kmat_sym_sum": [_vp, _i64, _ksp, _vp, _vp, _i64, ctypes.c_int, _vp],
+    "tgp_kmat_cross_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _i64, _vp],
+    "tgp_loglike_sum": [_vp, _vp, _vp, _i64, _ksp, _vp, _i64, _vp, ctypes.c_int, _vp, _vp, _vp, _i64, _vp],
+    "tgp_loglike_grad_sum_work_doubles": [_i64, _i32],
+    "tgp_loglike_grad_sum": [_vp, _vp, _vp, _i64, _ksp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
+    "tgp_predict_mean_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _vp, _vp],
+    "tgp_predict_mean_trunc_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _vp, _vp, _vp],
+    "tgp_predict_var_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -81,7 +99,7 @@ SIGNATURES = {
     "tgp_microbench_fp64": [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)],
 }
 _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctypes.c_int64,
-             "tgp_selinv_work_doubles": ctypes.c_int64,
+             "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 

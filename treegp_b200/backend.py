@@ -8,7 +8,7 @@ import numpy as np
 import torch
 
 from . import _cabi
-from ._cabi import TgpKernel, check
+from ._cabi import TgpKernel, TgpKernelSum, check
 
 F64 = torch.float64
 
@@ -66,16 +66,23 @@ def _check_dims(kdesc, X, Xs=None):
         raise ValueError("XA and XB must have the same number of columns (%d vs %d)" % (Xs.shape[1], X.shape[1]))
 
 
+def is_sum(kdesc):
+    """True for a TgpKernelSum (the *_sum entry points), False for a single-term TgpKernel."""
+    return isinstance(kdesc, TgpKernelSum)
+
+
 def kmat_sym(X, kdesc, diag_add=None, out=None, lower_only=False):
-    """K(X,X) + diag(diag_add).  Returns the (N, ld) workspace; the matrix is out[:, :N]."""
+    """K(X,X) + diag(diag_add).  Returns the (N, ld) workspace; the matrix is out[:, :N].  kdesc: TgpKernel or
+    TgpKernelSum (every function here that takes a descriptor accepts both)."""
     X = as_points(X)
     _check_dims(kdesc, X)
     N = X.shape[0]
     if out is None:
         out = alloc_matrix(N, N, X.device)
     lib = _cabi.load()
-    check(lib.tgp_kmat_sym(_p(X), N, ctypes.byref(kdesc), _p(diag_add), _p(out), out.stride(0),
-                           int(bool(lower_only)), _stream()), "tgp_kmat_sym")
+    fn = lib.tgp_kmat_sym_sum if is_sum(kdesc) else lib.tgp_kmat_sym
+    check(fn(_p(X), N, ctypes.byref(kdesc), _p(diag_add), _p(out), out.stride(0), int(bool(lower_only)), _stream()),
+          fn.__name__)
     return out
 
 
@@ -86,8 +93,8 @@ def kmat_cross(Xs, X, kdesc, out=None):
     if out is None:
         out = alloc_matrix(M, N, X.device)
     lib = _cabi.load()
-    check(lib.tgp_kmat_cross(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(out), out.stride(0), _stream()),
-          "tgp_kmat_cross")
+    fn = lib.tgp_kmat_cross_sum if is_sum(kdesc) else lib.tgp_kmat_cross
+    check(fn(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(out), out.stride(0), _stream()), fn.__name__)
     return out
 
 
@@ -214,7 +221,12 @@ def loglike(X, y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
     alpha = torch.empty(N, dtype=F64, device=X.device)
     out = torch.zeros(3, dtype=F64, device=X.device)
     info = torch.zeros(1, dtype=torch.int32, device=X.device)
-    if row_end is None:
+    if is_sum(kdesc):
+        re = None if row_end is None else _host_i64(row_end)
+        check(_cabi.load().tgp_loglike_sum(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
+                                           _p(alpha), int(bool(want_alpha)), _p(out), _p(info), re,
+                                           0 if row_end is None else len(row_end), _stream()), "tgp_loglike_sum")
+    elif row_end is None:
         check(_cabi.load().tgp_loglike(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
                                        _p(alpha), int(bool(want_alpha)), _p(out), _p(info), _stream()), "tgp_loglike")
     else:
@@ -252,7 +264,8 @@ def selinv_flops(row_end, n):
 def loglike_grad(X, y, yerr2, kdesc, work=None, row_end=None):
     """Log-likelihood and its gradient in one call (tgp_loglike_grad).  Returns (out[7] = logL, chi2, logdet,
     d logL / d ln amp, d logL / d m00, d m01, d m11; info; alpha = K^-1 y; work, which holds Z = K^-1 inside the
-    envelope afterwards).  row_end as for loglike (X, y, yerr2 sorted along the envelope's axis)."""
+    envelope afterwards).  row_end as for loglike (X, y, yerr2 sorted along the envelope's axis).  For a sum
+    (tgp_loglike_grad_sum) out has 4 + 4 nterms entries: the four derivatives per term, then d logL / d ln white."""
     X = as_points(X)
     _check_dims(kdesc, X)
     N = X.shape[0]
@@ -261,13 +274,20 @@ def loglike_grad(X, y, yerr2, kdesc, work=None, row_end=None):
     if work.shape[0] < N + 1:
         raise ValueError("loglike_grad workspace needs N+1 rows")
     alpha = torch.empty(N, dtype=F64, device=X.device)
-    out = torch.zeros(7, dtype=F64, device=X.device)
     info = torch.zeros(1, dtype=torch.int32, device=X.device)
-    scratch = _selinv_scratch(N, X.device)
+    lib = _cabi.load()
+    if is_sum(kdesc):
+        out = torch.zeros(4 + 4 * kdesc.nterms, dtype=F64, device=X.device)
+        scratch = torch.empty(int(lib.tgp_loglike_grad_sum_work_doubles(int(N), int(kdesc.nterms))), dtype=F64,
+                              device=X.device)
+        fn = lib.tgp_loglike_grad_sum
+    else:
+        out = torch.zeros(7, dtype=F64, device=X.device)
+        scratch = _selinv_scratch(N, X.device)
+        fn = lib.tgp_loglike_grad
     re = None if row_end is None else _host_i64(row_end)
-    check(_cabi.load().tgp_loglike_grad(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
-                                        _p(alpha), _p(out), _p(info), re, 0 if row_end is None else len(row_end),
-                                        _p(scratch), _stream()), "tgp_loglike_grad")
+    check(fn(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0), _p(alpha), _p(out), _p(info),
+             re, 0 if row_end is None else len(row_end), _p(scratch), _stream()), fn.__name__)
     return out, info, alpha, work
 
 
@@ -289,8 +309,8 @@ def predict_mean(Xs, X, kdesc, alpha, out=None, truncate=None):
     if truncate is None:
         truncate = M >= TRUNC_MIN_M and N >= TRUNC_MIN_N
     if not truncate:
-        check(lib.tgp_predict_mean(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(alpha), _p(out), _stream()),
-              "tgp_predict_mean")
+        fn = lib.tgp_predict_mean_sum if is_sum(kdesc) else lib.tgp_predict_mean
+        check(fn(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(alpha), _p(out), _stream()), fn.__name__)
         return out
     two_d = X.shape[1] == 2
     zt, zs = torch.zeros(N, dtype=F64, device=X.device), torch.zeros(M, dtype=F64, device=X.device)
@@ -299,8 +319,8 @@ def predict_mean(Xs, X, kdesc, alpha, out=None, truncate=None):
     Xt, at, Xss = X[ot].contiguous(), alpha[ot].contiguous(), Xs[os_].contiguous()
     work = torch.empty(int(lib.tgp_predict_work_doubles(N)), dtype=F64, device=X.device)
     tmp = torch.empty(M, dtype=F64, device=X.device)
-    check(lib.tgp_predict_mean_trunc(_p(Xss), M, _p(Xt), N, ctypes.byref(kdesc), _p(at), _p(tmp), _p(work),
-                                     _stream()), "tgp_predict_mean_trunc")
+    fn = lib.tgp_predict_mean_trunc_sum if is_sum(kdesc) else lib.tgp_predict_mean_trunc
+    check(fn(_p(Xss), M, _p(Xt), N, ctypes.byref(kdesc), _p(at), _p(tmp), _p(work), _stream()), fn.__name__)
     out[os_] = tmp
     return out
 
@@ -327,7 +347,8 @@ def knn_mean(X0, y0, Xq, k):
 
 
 def predict_var(Xs, X, kdesc, L, chunk=None, out=None, work=None, row_end=None):
-    """Diagonal predictive variance amp - |L^-1 k*|^2 (tgp_predict_var); row_end: the factor's envelope, X in the
+    """Diagonal predictive variance amp - |L^-1 k*|^2 (tgp_predict_var; a sum: sum_c amp_c + white - |L^-1 k*|^2,
+    tgp_predict_var_sum); row_end: the factor's envelope, X in the
     factor's (sorted) order (tgp_predict_var_env)."""
     Xs, X = as_points(Xs), as_points(X)
     _check_dims(kdesc, X, Xs)
@@ -340,7 +361,12 @@ def predict_var(Xs, X, kdesc, L, chunk=None, out=None, work=None, row_end=None):
         work = torch.empty(chunk * (N + 1), dtype=F64, device=X.device)
     if out is None:
         out = torch.empty(M, dtype=F64, device=X.device)
-    if row_end is None:
+    if is_sum(kdesc):
+        check(_cabi.load().tgp_predict_var_sum(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(L), L.stride(0),
+                                               None if row_end is None else _host_i64(row_end),
+                                               0 if row_end is None else len(row_end), _p(work), chunk, _p(out),
+                                               _stream()), "tgp_predict_var_sum")
+    elif row_end is None:
         check(_cabi.load().tgp_predict_var(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(L), L.stride(0), _p(work),
                                            chunk, _p(out), _stream()), "tgp_predict_var")
     else:
@@ -359,7 +385,10 @@ def var_chunk(N, M):
 def support_cutoffs(kdesc):
     """Per axis, the coordinate difference beyond which the kernel is below 1e-40 of its amplitude whatever the
     other coordinate: q = d^T M d >= d_a^2 / (M^-1)_aa, and f(q) <= 1e-40 for q >= tgp_profile_qcut(family).
-    NaN / inf for a metric that is not positive definite (callers then keep the dense path)."""
+    NaN / inf for a metric that is not positive definite (callers then keep the dense path).  A sum: per axis the
+    largest cut-off of its terms (the white level has no off-diagonal support)."""
+    if is_sum(kdesc):
+        return [float(v) for v in np.max([support_cutoffs(kdesc.term[c]) for c in range(kdesc.nterms)], axis=0)]
     qcut = float(_cabi.load().tgp_profile_qcut(int(kdesc.family)))
     with np.errstate(invalid="ignore", divide="ignore"):
         if kdesc.ndim == 1:

@@ -1344,15 +1344,19 @@ sumsq_kernel(const double* __restrict__ w, int64_t N, double* __restrict__ out1)
   }
 }
 
-static int loglike_impl(const double* X, const double* y, const double* yerr2, int64_t N,
-                        const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
-                        double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
+static int loglike_args(const double* X, const double* y, int64_t N, const double* work, const double* alpha,
+                        const double* out, const int32_t* info, const int64_t* row_end, int64_t nblocks) {
   TGP_CHECK_ARG(N > 0 && X && y && work && alpha && out && info, "null pointer / N");
   TGP_CHECK_ARG(row_end == nullptr || !check_envelope(row_end, nblocks, N),
                 "row_end must hold one entry per tgp_envelope_block() columns");
+  return TGP_OK;
+}
+
+// Everything after the K build (lower triangle of K + diag in `work`): factorisation, sweeps, reductions.
+static int loglike_after_build(const double* y, int64_t N, double* work, int64_t ld, double* alpha, int want_alpha,
+                               double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  int rc = tgp_kmat_sym(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
-  if (rc) return rc;
+  int rc;
   // out[1], out[2] double as scratch {logdet, chi2} until the finishing kernel reorders them
   double* tmp = out + 1;
   if (row_end) {
@@ -1390,6 +1394,16 @@ static int loglike_impl(const double* X, const double* y, const double* yerr2, i
   return TGP_OK;
 }
 
+static int loglike_impl(const double* X, const double* y, const double* yerr2, int64_t N,
+                        const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
+                        double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
+  int rc = loglike_args(X, y, N, work, alpha, out, info, row_end, nblocks);
+  if (rc) return rc;
+  rc = tgp_kmat_sym(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
+  if (rc) return rc;
+  return loglike_after_build(y, N, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+}
+
 extern "C" int tgp_loglike(const double* X, const double* y, const double* yerr2, int64_t N,
                            const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
                            double* out, int32_t* info, void* stream) {
@@ -1401,4 +1415,14 @@ extern "C" int tgp_loglike_env(const double* X, const double* y, const double* y
                                double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
   TGP_CHECK_ARG(row_end != nullptr, "row_end");
   return loglike_impl(X, y, yerr2, N, k, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+}
+
+extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N,
+                               const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
+                               double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
+  int rc = loglike_args(X, y, N, work, alpha, out, info, row_end, nblocks);
+  if (rc) return rc;
+  rc = tgp_kmat_sym_sum(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
+  if (rc) return rc;
+  return loglike_after_build(y, N, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
 }

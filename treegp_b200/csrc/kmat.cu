@@ -14,6 +14,7 @@
 #include <stdarg.h>
 #include <string.h>
 #include "tgp_common.cuh"
+#include "profile_policy.cuh"
 
 // ---- error state / misc host helpers --------------------------------------------------------
 static thread_local char g_err[512] = "";
@@ -64,14 +65,14 @@ __device__ __forceinline__ void store2(double* p, double a, double b, bool vec, 
 }
 
 // Symmetric build.  Grid: one CTA per lower-triangular tile pair (I >= J), linearised.
-template <int FAM>
+template <class P>
 __global__ void __launch_bounds__(KT_THREADS)
-kmat_sym_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double* __restrict__ diag_add,
+kmat_sym_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ diag_add,
                 double* __restrict__ out, int64_t ld, int lower_only, int vec_ok,
                 const double* __restrict__ phi_g) {
   __shared__ double xr[KT], yr[KT], xc[KT], yc[KT];
   __shared__ double tile[KT * KT_PITCH];
-  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  __shared__ double phi_s[P::kPhiSize];
 
   // linear tile id -> (I, J), I >= J
   const int64_t t = blockIdx.x;
@@ -82,18 +83,18 @@ kmat_sym_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double*
   const int64_t r0 = I * KT, c0 = J * KT;
   const int tid = threadIdx.x;
 
-  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   if (tid < KT) {
     const int64_t r = r0 + tid;
     const bool ok = r < N;
-    xr[tid] = ok ? X[r * kd.ndim] : 0.0;
-    yr[tid] = (ok && kd.ndim == 2) ? X[r * 2 + 1] : 0.0;
+    xr[tid] = ok ? X[r * prof.desc.ndim] : 0.0;
+    yr[tid] = (ok && prof.desc.ndim == 2) ? X[r * 2 + 1] : 0.0;
   } else if (tid < 2 * KT) {
     const int l = tid - KT;
     const int64_t c = c0 + l;
     const bool ok = c < N;
-    xc[l] = ok ? X[c * kd.ndim] : 0.0;
-    yc[l] = (ok && kd.ndim == 2) ? X[c * 2 + 1] : 0.0;
+    xc[l] = ok ? X[c * prof.desc.ndim] : 0.0;
+    yc[l] = (ok && prof.desc.ndim == 2) ? X[c * 2 + 1] : 0.0;
   }
   __syncthreads();
 
@@ -107,21 +108,13 @@ kmat_sym_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double*
   // von Karman: the profile (series / per-binade polynomial, sqrt, cbrt, exp) is ~350 instructions per evaluation;
   // unrolled 8 x 2 times the kernel was 94 KB of SASS and stalled on instruction fetch (no_instruction 4.4 per
   // issue, profiles/r2_start_kmat_vk.ncu.txt) -- two rows per trip keep it inside the instruction cache
-#pragma unroll(FAM == TGP_FAM_VONKARMAN ? 2 : KT / 8)
+#pragma unroll(P::kHeavy ? 2 : KT / 8)
   for (int rr = 0; rr < KT / 8; ++rr) {
     const int rl = warp + 8 * rr;
     const int64_t rg = r0 + rl;
     const double rx = xr[rl], ry = yr[rl];
-    const double q0 = tgp_qform(kd, rx - cx0, ry - cy0), q1 = tgp_qform(kd, rx - cx1, ry - cy1);
-    double v0 = kd.amp * tgp_profile<FAM>(q0, phi_s);
-    double v1 = kd.amp * tgp_profile<FAM>(q1, phi_s);
-    if (FAM == TGP_FAM_VONKARMAN) {
-      // Reference quirk kept for parity: in K(X,X) the von Karman kernels leave OFF-diagonal entries of
-      // coincident points at 0 (pdist == 0 is filtered out and only the diagonal is refilled,
-      // kernels.py:253-262 and :360-367); K(X,Y) returns amp there (kernels.py:273-276, :378-381).
-      if (q0 == 0.0 && rg != cg) v0 = 0.0;
-      if (q1 == 0.0 && rg != cg + 1) v1 = 0.0;
-    }
+    double v0, v1;
+    prof.sym2(rx, ry, cx0, cy0, cx1, cy1, rg, cg, phi_s, v0, v1);
     if (diag_tile && diag_add != nullptr) {
       if (rg == cg && rg < N) v0 += diag_add[rg];
       if (rg == cg + 1 && rg < N) v1 += diag_add[rg];
@@ -158,41 +151,41 @@ kmat_sym_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double*
 }
 
 // Rectangular build K(Xs, X): rows = test points, columns = training points.
-template <int FAM>
+template <class P>
 __global__ void __launch_bounds__(KT_THREADS)
 kmat_cross_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
-                  KDesc kd, double* __restrict__ out, int64_t ld, int vec_ok,
+                  P prof, double* __restrict__ out, int64_t ld, int vec_ok,
                   const double* __restrict__ phi_g) {
   __shared__ double xr[KT], yr[KT], xc[KT], yc[KT];
-  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  __shared__ double phi_s[P::kPhiSize];
   const int64_t r0 = (int64_t)blockIdx.x * KT, c0 = (int64_t)blockIdx.y * KT;
   const int tid = threadIdx.x;
-  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   if (tid < KT) {
     const int64_t r = r0 + tid;
     const bool ok = r < M;
-    xr[tid] = ok ? Xs[r * kd.ndim] : 0.0;
-    yr[tid] = (ok && kd.ndim == 2) ? Xs[r * 2 + 1] : 0.0;
+    xr[tid] = ok ? Xs[r * prof.desc.ndim] : 0.0;
+    yr[tid] = (ok && prof.desc.ndim == 2) ? Xs[r * 2 + 1] : 0.0;
   } else if (tid < 2 * KT) {
     const int l = tid - KT;
     const int64_t c = c0 + l;
     const bool ok = c < N;
-    xc[l] = ok ? X[c * kd.ndim] : 0.0;
-    yc[l] = (ok && kd.ndim == 2) ? X[c * 2 + 1] : 0.0;
+    xc[l] = ok ? X[c * prof.desc.ndim] : 0.0;
+    yc[l] = (ok && prof.desc.ndim == 2) ? X[c * 2 + 1] : 0.0;
   }
   __syncthreads();
   const int lane = tid & 31, warp = tid >> 5;
   const int cl = 2 * lane;
   const double cx0 = xc[cl], cy0 = yc[cl], cx1 = xc[cl + 1], cy1 = yc[cl + 1];
   const int64_t cg = c0 + cl;
-#pragma unroll(FAM == TGP_FAM_VONKARMAN ? 2 : KT / 8)
+#pragma unroll(P::kHeavy ? 2 : KT / 8)
   for (int rr = 0; rr < KT / 8; ++rr) {
     const int rl = warp + 8 * rr;
     const int64_t rg = r0 + rl;
     if (rg >= M) continue;
     const double rx = xr[rl], ry = yr[rl];
-    const double v0 = kd.amp * tgp_profile<FAM>(tgp_qform(kd, rx - cx0, ry - cy0), phi_s);
-    const double v1 = kd.amp * tgp_profile<FAM>(tgp_qform(kd, rx - cx1, ry - cy1), phi_s);
+    double v0, v1;
+    prof.cross2(rx, ry, cx0, cy0, cx1, cy1, phi_s, v0, v1);
     const bool ok0 = cg < N, ok1 = cg + 1 < N;
     store2(out + rg * ld + cg, v0, v1, vec_ok && ok0, ok0, ok1);
   }
@@ -212,8 +205,8 @@ extern "C" int tgp_kmat_sym(const double* X, int64_t N, const tgp_kernel* k, con
   const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
   cudaStream_t st = (cudaStream_t)stream;
   const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (kmat_sym_kernel<FAM><<<(unsigned)ntiles, KT_THREADS, 0, st>>>(
-                                   X, N, kd, diag_add, out, ld, lower_only, vec_ok, phi)));
+  TGP_FAMILY_SWITCH(k->family, (kmat_sym_kernel<FamilyProfile<FAM>><<<(unsigned)ntiles, KT_THREADS, 0, st>>>(
+                                   X, N, FamilyProfile<FAM>{kd}, diag_add, out, ld, lower_only, vec_ok, phi)));
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }
@@ -230,8 +223,42 @@ extern "C" int tgp_kmat_cross(const double* Xs, int64_t M, const double* X, int6
   TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
   cudaStream_t st = (cudaStream_t)stream;
   const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (kmat_cross_kernel<FAM><<<grid, KT_THREADS, 0, st>>>(
-                                   Xs, M, X, N, kd, out, ld, vec_ok, phi)));
+  TGP_FAMILY_SWITCH(k->family, (kmat_cross_kernel<FamilyProfile<FAM>><<<grid, KT_THREADS, 0, st>>>(
+                                   Xs, M, X, N, FamilyProfile<FAM>{kd}, out, ld, vec_ok, phi)));
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+extern "C" int tgp_kmat_sym_sum(const double* X, int64_t N, const tgp_kernel_sum* k, const double* diag_add,
+                                double* out, int64_t ld, int lower_only, void* stream) {
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  if (k->nterms == 1 && k->white == 0.0)   // one term: the single-term kernel, bit for bit
+    return tgp_kmat_sym(X, N, &k->term[0], diag_add, out, ld, lower_only, stream);
+  TGP_CHECK_ARG(N >= 0 && ld >= N, "N/ld");
+  if (N == 0) return TGP_OK;
+  TGP_CHECK_ARG(X && out, "null pointer");
+  const int64_t nt = tgp_cdiv(N, KT);
+  const int64_t ntiles = nt * (nt + 1) / 2;
+  TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
+  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
+  kmat_sym_kernel<SumProfile><<<(unsigned)ntiles, KT_THREADS, 0, (cudaStream_t)stream>>>(
+      X, N, SumProfile{make_ksumdesc(k)}, diag_add, out, ld, lower_only, vec_ok, tgp_phi_device());
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+extern "C" int tgp_kmat_cross_sum(const double* Xs, int64_t M, const double* X, int64_t N,
+                                  const tgp_kernel_sum* k, double* out, int64_t ld, void* stream) {
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  if (k->nterms == 1) return tgp_kmat_cross(Xs, M, X, N, &k->term[0], out, ld, stream);   // no white in K(Xs, X)
+  TGP_CHECK_ARG(M >= 0 && N >= 0 && ld >= N, "M/N/ld");
+  if (M == 0 || N == 0) return TGP_OK;
+  TGP_CHECK_ARG(Xs && X && out, "null pointer");
+  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
+  dim3 grid((unsigned)tgp_cdiv(M, KT), (unsigned)tgp_cdiv(N, KT));
+  TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
+  kmat_cross_kernel<SumProfile><<<grid, KT_THREADS, 0, (cudaStream_t)stream>>>(
+      Xs, M, X, N, SumProfile{make_ksumdesc(k)}, out, ld, vec_ok, tgp_phi_device());
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

@@ -5,6 +5,7 @@
 // matrix HT (320 GB at M = 1e6, N = 4e4); here each thread owns one test point, the training
 // coordinates and alpha stream through shared memory, and only M doubles are written.
 #include "tgp_common.cuh"
+#include "profile_policy.cuh"
 
 constexpr int PM_THREADS = 256;   // test points per CTA
 constexpr int PM_TILE = 1024;     // training points per shared-memory tile
@@ -12,20 +13,20 @@ constexpr int PM_TILE = 1024;     // training points per shared-memory tile
 // grid: (ceil(M / PM_THREADS), nsplit).  Split s handles training tiles s, s + nsplit, ...
 // nsplit == 1 writes mean directly; otherwise partial sums are added with red.global.add.f64 into a
 // zeroed output (used only when M alone cannot fill the machine).
-template <int FAM>
+template <class P>
 __global__ void __launch_bounds__(PM_THREADS)
 predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
-                    KDesc kd, const double* __restrict__ alpha, double* __restrict__ mean,
+                    P prof, const double* __restrict__ alpha, double* __restrict__ mean,
                     const double* __restrict__ phi_g) {
   __shared__ double2 pxy[PM_TILE];
   __shared__ double pa[PM_TILE];
-  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  __shared__ double phi_s[P::kPhiSize];
   const int tid = threadIdx.x;
-  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   const int64_t m = (int64_t)blockIdx.x * PM_THREADS + tid;
   const bool live = m < M;
-  const double sx = live ? Xs[m * kd.ndim] : 0.0;
-  const double sy = (live && kd.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
+  const double sx = live ? Xs[m * prof.desc.ndim] : 0.0;
+  const double sy = (live && prof.desc.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
   const int nsplit = gridDim.y;
   const int64_t ntile = (N + PM_TILE - 1) / PM_TILE;
   double acc0 = 0.0, acc1 = 0.0;
@@ -36,19 +37,24 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
       const int64_t n = n0 + i;
       const bool ok = n < N;
       double2 p;
-      p.x = ok ? X[n * kd.ndim] : 0.0;
-      p.y = (ok && kd.ndim == 2) ? X[n * 2 + 1] : 0.0;
+      p.x = ok ? X[n * prof.desc.ndim] : 0.0;
+      p.y = (ok && prof.desc.ndim == 2) ? X[n * 2 + 1] : 0.0;
       pxy[i] = p;
-      pa[i] = ok ? kd.amp * alpha[n] : 0.0;  // padded points carry zero weight
+      pa[i] = ok ? prof.weight() * alpha[n] : 0.0;  // padded points carry zero weight
     }
     __syncthreads();
+    if constexpr (P::kSum) {
+      for (int i = 0; i < PM_TILE; i += 2) prof.mean2(sx, sy, pxy, pa, i, phi_s, acc0, acc1);
+    } else {
+      const KDesc& kd = prof.desc;
 #pragma unroll 2
-    for (int i = 0; i < PM_TILE; i += 2) {
-      const double2 p0 = pxy[i], p1 = pxy[i + 1];
-      const double q0 = tgp_qform(kd, sx - p0.x, sy - p0.y);
-      const double q1 = tgp_qform(kd, sx - p1.x, sy - p1.y);
-      acc0 = fma(tgp_profile<FAM>(q0, phi_s), pa[i], acc0);
-      acc1 = fma(tgp_profile<FAM>(q1, phi_s), pa[i + 1], acc1);
+      for (int i = 0; i < PM_TILE; i += 2) {
+        const double2 p0 = pxy[i], p1 = pxy[i + 1];
+        const double q0 = tgp_qform(kd, sx - p0.x, sy - p0.y);
+        const double q1 = tgp_qform(kd, sx - p1.x, sy - p1.y);
+        acc0 = fma(tgp_profile<P::kFam>(q0, phi_s), pa[i], acc0);
+        acc1 = fma(tgp_profile<P::kFam>(q1, phi_s), pa[i + 1], acc1);
+      }
     }
   }
   if (live) {
@@ -58,14 +64,13 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
   }
 }
 
-extern "C" int tgp_predict_mean(const double* Xs, int64_t M, const double* X, int64_t N,
-                                const tgp_kernel* k, const double* alpha, double* mean, void* stream) {
-  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+template <class P>
+static int predict_mean_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof,
+                               const double* alpha, double* mean, void* stream) {
   TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
   if (M == 0) return TGP_OK;
   TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha)), "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
-  const KDesc kd = make_kdesc(k);
   const int64_t gx = tgp_cdiv(M, PM_THREADS);
   const int64_t ntile = tgp_cdiv(N, PM_TILE);
   int64_t nsplit = 1;
@@ -76,11 +81,24 @@ extern "C" int tgp_predict_mean(const double* Xs, int64_t M, const double* X, in
   if (nsplit > 1 || N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * sizeof(double), st));
   if (N == 0) return TGP_OK;
   dim3 grid((unsigned)gx, (unsigned)nsplit);
-  const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (predict_mean_kernel<FAM><<<grid, PM_THREADS, 0, st>>>(Xs, M, X, N, kd, alpha,
-                                                                                     mean, phi)));
+  predict_mean_kernel<P><<<grid, PM_THREADS, 0, st>>>(Xs, M, X, N, prof, alpha, mean, tgp_phi_device());
   TGP_LAUNCH_CHECK();
   return TGP_OK;
+}
+
+extern "C" int tgp_predict_mean(const double* Xs, int64_t M, const double* X, int64_t N,
+                                const tgp_kernel* k, const double* alpha, double* mean, void* stream) {
+  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+  const KDesc kd = make_kdesc(k);
+  TGP_FAMILY_SWITCH(k->family, return predict_mean_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, alpha, mean, stream));
+  return TGP_OK;
+}
+
+extern "C" int tgp_predict_mean_sum(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
+                                    const double* alpha, double* mean, void* stream) {
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  if (k->nterms == 1) return tgp_predict_mean(Xs, M, X, N, &k->term[0], alpha, mean, stream);
+  return predict_mean_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, alpha, mean, stream);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -136,24 +154,24 @@ point_boxes_kernel(const double* __restrict__ X, int64_t N, int ndim, double* __
   }
 }
 
-template <int FAM>
+template <class P>
 __global__ void __launch_bounds__(PM_THREADS)
 predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
-                          KDesc kd, const double* __restrict__ alpha, double* __restrict__ mean,
+                          P prof, const double* __restrict__ alpha, double* __restrict__ mean,
                           const double* __restrict__ phi_g, const double* __restrict__ boxes, int64_t ngroups,
                           double r2cut) {
   __shared__ double2 pxy[PG];
   __shared__ double pa[PG];
-  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  __shared__ double phi_s[P::kPhiSize];
   __shared__ double red[8][4];
   __shared__ int list[PM_THREADS];
   __shared__ int wcount[8];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   const int64_t m = (int64_t)blockIdx.x * PM_THREADS + tid;
   const bool live = m < M;
-  const double sx = live ? Xs[m * kd.ndim] : 0.0;
-  const double sy = (live && kd.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
+  const double sx = live ? Xs[m * prof.desc.ndim] : 0.0;
+  const double sy = (live && prof.desc.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
   // bounding box of this CTA's test points
   double bx0 = live ? sx : INFINITY, bx1 = live ? sx : -INFINITY, by0 = live ? sy : INFINITY, by1 = live ? sy : -INFINITY;
 #pragma unroll
@@ -200,56 +218,98 @@ predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double
         const int64_t n = n0 + tid;
         const bool ok = n < N;
         double2 p;
-        p.x = ok ? X[n * kd.ndim] : 0.0;
-        p.y = (ok && kd.ndim == 2) ? X[n * 2 + 1] : 0.0;
+        p.x = ok ? X[n * prof.desc.ndim] : 0.0;
+        p.y = (ok && prof.desc.ndim == 2) ? X[n * 2 + 1] : 0.0;
         pxy[tid] = p;
-        pa[tid] = ok ? kd.amp * alpha[n] : 0.0;
+        pa[tid] = ok ? prof.weight() * alpha[n] : 0.0;
       }
       __syncthreads();
+      if constexpr (P::kSum) {
+        for (int i = 0; i < PG; i += 2) prof.mean2(sx, sy, pxy, pa, i, phi_s, acc0, acc1);
+      } else {
 #pragma unroll 2
-      for (int i = 0; i < PG; i += 2) {
-        const double2 p0 = pxy[i], p1 = pxy[i + 1];
-        const double q0 = tgp_qform(kd, sx - p0.x, sy - p0.y);
-        const double q1 = tgp_qform(kd, sx - p1.x, sy - p1.y);
-        acc0 = fma(tgp_profile<FAM>(q0, phi_s), pa[i], acc0);
-        acc1 = fma(tgp_profile<FAM>(q1, phi_s), pa[i + 1], acc1);
+        for (int i = 0; i < PG; i += 2) {
+          const double2 p0 = pxy[i], p1 = pxy[i + 1];
+          const double q0 = tgp_qform(prof.desc, sx - p0.x, sy - p0.y);
+          const double q1 = tgp_qform(prof.desc, sx - p1.x, sy - p1.y);
+          acc0 = fma(tgp_profile<P::kFam>(q0, phi_s), pa[i], acc0);
+          acc1 = fma(tgp_profile<P::kFam>(q1, phi_s), pa[i + 1], acc1);
+        }
       }
     }
   }
   if (live) mean[m] = acc0 + acc1;
 }
 
-extern "C" int tgp_predict_mean_trunc(const double* Xs, int64_t M, const double* X, int64_t N,
-                                      const tgp_kernel* k, const double* alpha, double* mean, double* work,
-                                      void* stream) {
-  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
-  TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
-  if (M == 0) return TGP_OK;
-  TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha && work)), "null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (N == 0) {
-    TGP_CUDA(cudaMemsetAsync(mean, 0, M * sizeof(double), st));
-    return TGP_OK;
-  }
-  const KDesc kd = make_kdesc(k);
-  // smallest eigenvalue of the inverse metric: q >= lmin |delta|^2
+// smallest eigenvalue of the inverse metric: q >= lmin |delta|^2
+static double metric_lmin(const tgp_kernel* k) {
   double lmin = k->m00;
   if (k->ndim == 2) {
     const double h = 0.5 * (k->m00 - k->m11);
     lmin = 0.5 * (k->m00 + k->m11) - sqrt(h * h + k->m01 * k->m01);
   }
-  TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
-  const double r2cut = profile_qcut(k->family) / lmin;
+  return lmin;
+}
+
+// r2cut: squared Euclidean distance beyond which every pair is below the cut-off (caller: > 0)
+template <class P>
+static int predict_mean_trunc_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof,
+                                     double r2cut, const double* alpha, double* mean, double* work, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
   const int64_t ngroups = tgp_cdiv(N, PG);
-  point_boxes_kernel<<<(unsigned)tgp_cdiv(ngroups, 8), 256, 0, st>>>(X, N, k->ndim, work, ngroups);
+  point_boxes_kernel<<<(unsigned)tgp_cdiv(ngroups, 8), 256, 0, st>>>(X, N, prof.desc.ndim, work, ngroups);
   TGP_LAUNCH_CHECK();
   const double* phi = tgp_phi_device();
   const int64_t gx = tgp_cdiv(M, PM_THREADS);
   TGP_CHECK_ARG(gx < (1ll << 31), "M too large for one launch");
-  TGP_FAMILY_SWITCH(k->family, (predict_mean_trunc_kernel<FAM><<<(unsigned)gx, PM_THREADS, 0, st>>>(
-                                   Xs, M, X, N, kd, alpha, mean, phi, work, ngroups, r2cut)));
+  predict_mean_trunc_kernel<P><<<(unsigned)gx, PM_THREADS, 0, st>>>(Xs, M, X, N, prof, alpha, mean, phi, work,
+                                                                      ngroups, r2cut);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
+}
+
+static int predict_mean_trunc_args(const double* Xs, int64_t M, const double* X, int64_t N, const double* alpha,
+                                   double* mean, double* work, void* stream) {
+  TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
+  if (M == 0) return TGP_OK;
+  TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha && work)), "null pointer");
+  if (N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * sizeof(double), (cudaStream_t)stream));
+  return TGP_OK;
+}
+
+extern "C" int tgp_predict_mean_trunc(const double* Xs, int64_t M, const double* X, int64_t N,
+                                      const tgp_kernel* k, const double* alpha, double* mean, double* work,
+                                      void* stream) {
+  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+  const int rc = predict_mean_trunc_args(Xs, M, X, N, alpha, mean, work, stream);
+  if (rc || M == 0 || N == 0) return rc;
+  const double lmin = metric_lmin(k);
+  TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
+  const double r2cut = profile_qcut(k->family) / lmin;
+  const KDesc kd = make_kdesc(k);
+  TGP_FAMILY_SWITCH(k->family, return predict_mean_trunc_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, r2cut, alpha,
+                                                                mean, work, stream));
+  return TGP_OK;
+}
+
+// A group is skipped only when it is beyond the cut-off of every term: the union of the supports is the largest
+// per-term qcut_c / lmin(M_c).  Each skipped pair is below 1e-40 |amp_c| for every term, so the mean changes by at
+// most 1e-40 sum_c |amp_c| sum_n |alpha_n|.
+extern "C" int tgp_predict_mean_trunc_sum(const double* Xs, int64_t M, const double* X, int64_t N,
+                                          const tgp_kernel_sum* k, const double* alpha, double* mean, double* work,
+                                          void* stream) {
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  if (k->nterms == 1) return tgp_predict_mean_trunc(Xs, M, X, N, &k->term[0], alpha, mean, work, stream);
+  const int rc = predict_mean_trunc_args(Xs, M, X, N, alpha, mean, work, stream);
+  if (rc || M == 0 || N == 0) return rc;
+  double r2cut = 0.0;
+  for (int c = 0; c < k->nterms; ++c) {
+    const double lmin = metric_lmin(&k->term[c]);
+    TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
+    const double r2 = profile_qcut(k->term[c].family) / lmin;
+    if (r2 > r2cut) r2cut = r2;
+  }
+  return predict_mean_trunc_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r2cut, alpha, mean, work, stream);
 }
 
 // var[m] = amp - sum_n V[m][n]^2, V = K(Xs, X) L^-T (row m = L^-1 k*_m).  Warp per row.
@@ -274,23 +334,31 @@ var_from_rows_kernel(const double* __restrict__ V, int64_t M, int64_t N, int64_t
   if (lane == 0) var[m] = amp - s;
 }
 
+// k or ks (the other NULL): single-term or sum kernel; the prior variance is amp, or sum_c amp_c + white
 static int predict_var_impl(const double* Xs, int64_t M, const double* X, int64_t N,
-                            const tgp_kernel* k, const double* L, int64_t ld, const int64_t* row_end,
-                            int64_t nblocks, double* work, int64_t chunk, double* var, void* stream) {
-  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+                            const tgp_kernel* k, const tgp_kernel_sum* ks, const double* L, int64_t ld,
+                            const int64_t* row_end, int64_t nblocks, double* work, int64_t chunk, double* var,
+                            void* stream) {
+  if (ks) TGP_CHECK_ARG(ksum_ok(ks), "kernel sum descriptor");
+  else TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
   TGP_CHECK_ARG(M >= 0 && N > 0 && ld >= N && chunk > 0, "shape");
   if (M == 0) return TGP_OK;
   TGP_CHECK_ARG(Xs && X && L && work && var, "null pointer");
   const int64_t ldw = (N + 1) & ~1ll;  // even row pitch for the DMMA operand loads
   TGP_CHECK_ARG(((uintptr_t)work % 16) == 0, "work must be 16-byte aligned");
+  const int ndim = ks ? ks->ndim : k->ndim;
+  double prior = ks ? ks->white : k->amp;
+  if (ks)
+    for (int c = 0; c < ks->nterms; ++c) prior += ks->term[c].amp;
   for (int64_t m0 = 0; m0 < M; m0 += chunk) {
     const int64_t mc = (M - m0 < chunk) ? (M - m0) : chunk;
-    int rc = tgp_kmat_cross(Xs + m0 * k->ndim, mc, X, N, k, work, ldw, stream);
+    int rc = ks ? tgp_kmat_cross_sum(Xs + m0 * ndim, mc, X, N, ks, work, ldw, stream)
+                : tgp_kmat_cross(Xs + m0 * ndim, mc, X, N, k, work, ldw, stream);
     if (rc) return rc;
     rc = row_end ? tgp_trsm_rows_env(L, N, ld, row_end, nblocks, work, mc, ldw, stream)
                  : tgp_trsm_rows(L, N, ld, work, mc, ldw, stream);
     if (rc) return rc;
-    var_from_rows_kernel<<<(unsigned)tgp_cdiv(mc, 8), 256, 0, (cudaStream_t)stream>>>(work, mc, N, ldw, k->amp,
+    var_from_rows_kernel<<<(unsigned)tgp_cdiv(mc, 8), 256, 0, (cudaStream_t)stream>>>(work, mc, N, ldw, prior,
                                                                                       var + m0);
     TGP_LAUNCH_CHECK();
   }
@@ -300,7 +368,7 @@ static int predict_var_impl(const double* Xs, int64_t M, const double* X, int64_
 extern "C" int tgp_predict_var(const double* Xs, int64_t M, const double* X, int64_t N,
                                const tgp_kernel* k, const double* L, int64_t ld, double* work,
                                int64_t chunk, double* var, void* stream) {
-  return predict_var_impl(Xs, M, X, N, k, L, ld, nullptr, 0, work, chunk, var, stream);
+  return predict_var_impl(Xs, M, X, N, k, nullptr, L, ld, nullptr, 0, work, chunk, var, stream);
 }
 
 // The same with a factor whose envelope is known (tgp_potrf_env): the multi-right-hand-side forward substitution
@@ -309,7 +377,14 @@ extern "C" int tgp_predict_var_env(const double* Xs, int64_t M, const double* X,
                                    const tgp_kernel* k, const double* L, int64_t ld, const int64_t* row_end,
                                    int64_t nblocks, double* work, int64_t chunk, double* var, void* stream) {
   TGP_CHECK_ARG(row_end != nullptr, "row_end");
-  return predict_var_impl(Xs, M, X, N, k, L, ld, row_end, nblocks, work, chunk, var, stream);
+  return predict_var_impl(Xs, M, X, N, k, nullptr, L, ld, row_end, nblocks, work, chunk, var, stream);
+}
+
+extern "C" int tgp_predict_var_sum(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
+                                   const double* L, int64_t ld, const int64_t* row_end, int64_t nblocks, double* work,
+                                   int64_t chunk, double* var, void* stream) {
+  TGP_CHECK_ARG(k != nullptr, "kernel sum descriptor");
+  return predict_var_impl(Xs, M, X, N, nullptr, k, L, ld, row_end, nblocks, work, chunk, var, stream);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -19,6 +19,7 @@
 #include <vector>
 #include "tgp_common.cuh"
 #include "profile_dq.cuh"
+#include "profile_policy.cuh"
 
 extern "C" int tgp_trsm_rows(const double* L, int64_t N, int64_t ld, double* B, int64_t M, int64_t ldb, void* stream);
 extern "C" int tgp_gemm_nt_sub(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
@@ -30,6 +31,9 @@ extern "C" int tgp_loglike_env(const double* X, const double* y, const double* y
                                double* work, int64_t ld, double* alpha, int want_alpha, double* out, int32_t* info,
                                const int64_t* row_end, int64_t nblocks, void* stream);
 extern "C" int tgp_envelope_block(void);
+extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N,
+                               const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
+                               double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream);
 
 constexpr int SB = 512;            // block columns of the recurrence: the envelope's block (tgp_envelope_block)
 constexpr int GT = 64;             // contraction tile edge
@@ -41,11 +45,19 @@ static int64_t grad_tiles(int64_t N) {
   return nt * (nt + 1) / 2;
 }
 
-extern "C" int64_t tgp_selinv_work_doubles(int64_t N) {
+// ncols partial sums per contraction tile: 4 for one term, 4 nterms + 1 for a sum
+static int64_t grad_work_doubles(int64_t N, int ncols) {
   if (N < 1) N = 1;
   const int64_t selinv = 2 * (int64_t)SB * SB + (int64_t)SB * even64(N);   // -W^T, W^T, T^T
-  const int64_t partials = 4 * grad_tiles(N);                               // contraction partial sums
+  const int64_t partials = ncols * grad_tiles(N);                           // contraction partial sums
   return (selinv > partials ? selinv : partials) + even64(tgp_cdiv(N, SB));  // + the device copy of row_end
+}
+
+extern "C" int64_t tgp_selinv_work_doubles(int64_t N) { return grad_work_doubles(N, 4); }
+
+extern "C" int64_t tgp_loglike_grad_sum_work_doubles(int64_t N, int32_t nterms) {
+  if (nterms < 1 || nterms > TGP_MAX_TERMS) return -1;
+  return grad_work_doubles(N, 4 * nterms + 1);
 }
 
 // ---- small helpers --------------------------------------------------------------------------------------------
@@ -185,14 +197,19 @@ extern "C" int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_e
 // 1e-36 for the von Karman profile (qcut = 224: |q f'| = pi sqrt(q) K_{1/6}/K_{5/6} f ~ 47 f) and below
 // sqrt(q)/2 f, sqrt(3q) f, 5/6 (1 + sqrt(5q)) sqrt(5q) f ~ 1e-37 for the Matern families -- every dropped term is
 // below 1e-36 a |w_ij| |dq / dm| / q.
-template <int FAM>
+//
+// Sums (SumProfile): CTA (t, c) contracts term c of tile t into columns 4 c .. 4 c + 3 of the tile's 4 nterms + 1
+// partials; the CTAs of term 0 also sum w_ii = alpha_i^2 - Z_ii over the diagonal, times the white level, into the
+// last column (d K / d ln white = white I).
+template <class P>
 __global__ void __launch_bounds__(GT_THREADS)
-grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const double* __restrict__ Z, int64_t ld,
+grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ Z, int64_t ld,
                      const double* __restrict__ alpha, const int64_t* __restrict__ re_dev,
                      double* __restrict__ partials, const double* __restrict__ phi_g) {
   __shared__ double xr[GT], yr[GT], ar[GT], xc[GT], yc[GT], ac[GT];
-  __shared__ double red[GT_THREADS / 32][4];
-  __shared__ double phi_s[FAM == TGP_FAM_VONKARMAN ? TGP_VK_PHI_SIZE : 1];
+  __shared__ double red[GT_THREADS / 32][P::kSum ? 5 : 4];
+  __shared__ double phi_s[P::kPhiSize];
+  const KDesc& kd = prof.grad_term();
   const int64_t t = blockIdx.x;
   int64_t I = (int64_t)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
   while (I * (I + 1) / 2 > t) --I;
@@ -202,10 +219,13 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const do
   const int64_t rend = re_dev ? re_dev[c0 / SB] : N;   // one past the last envelope row of this block column
   const int tid = threadIdx.x;
   if (r0 >= rend) {
-    if (tid < 4) partials[4 * t + tid] = 0.0;
+    if (tid < 4) partials[prof.partial(t, tid)] = 0.0;
+    if constexpr (P::kSum) {
+      if (tid == 4 && blockIdx.y == 0) partials[prof.white_partial(t)] = 0.0;
+    }
     return;
   }
-  if (FAM == TGP_FAM_VONKARMAN) tgp_stage_phi(phi_s, phi_g);
+  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   if (tid < GT) {
     const int64_t r = r0 + tid;
     const bool ok = r < N;
@@ -223,7 +243,8 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const do
   __syncthreads();
   const int lane = tid & 31, warp = tid >> 5;
   double s[4] = {0.0, 0.0, 0.0, 0.0};
-#pragma unroll(FAM == TGP_FAM_VONKARMAN ? 1 : GT / 8)
+  double sw = 0.0;   // sums: the white column
+#pragma unroll(P::kHeavy ? 1 : GT / 8)
   for (int rr = 0; rr < GT / 8; ++rr) {
     const int rl = warp + 8 * rr;
     const int64_t rg = r0 + rl;
@@ -236,12 +257,15 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const do
       const double dx = xr[rl] - xc[cl], dy = yr[rl] - yc[cl];
       const double q = tgp_qform(kd, dx, dy);
       const double wij = (rg == cg ? 1.0 : 2.0) * (ar[rl] * ac[cl] - Z[rg * ld + cg]);
-      double f = tgp_profile<FAM>(q, phi_s);
+      double f = prof.f(kd, q, phi_s);
       // K(X, X) of the von Karman kernels is 0 between distinct coincident points (kmat.cu, kernels.py:253-262)
-      if (FAM == TGP_FAM_VONKARMAN && q == 0.0 && rg != cg) f = 0.0;
+      if (prof.vk(kd) && q == 0.0 && rg != cg) f = 0.0;
+      if constexpr (P::kSum) {
+        if (rg == cg) sw += wij;
+      }
       s[0] = fma(wij, kd.amp * f, s[0]);
       if (q > 0.0) {
-        const double d = wij * kd.amp * tgp_profile_dq<FAM>(q, phi_s);
+        const double d = wij * kd.amp * prof.fdq(kd, q, phi_s);
         s[1] = fma(d, dx * dx, s[1]);
         s[2] = fma(d, 2.0 * dx * dy, s[2]);
         s[3] = fma(d, dy * dy, s[3]);
@@ -253,6 +277,11 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const do
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s[c] += __shfl_xor_sync(0xffffffffu, s[c], o);
   }
+  if constexpr (P::kSum) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) sw += __shfl_xor_sync(0xffffffffu, sw, o);
+    if (lane == 0) red[warp][4] = sw;
+  }
   if (lane == 0) {
 #pragma unroll
     for (int c = 0; c < 4; ++c) red[warp][c] = s[c];
@@ -261,68 +290,120 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, KDesc kd, const do
   if (tid < 4) {
     double v = 0.0;
     for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi][tid];
-    partials[4 * t + tid] = v;
+    partials[prof.partial(t, tid)] = v;
+  }
+  if constexpr (P::kSum) {
+    if (tid == 4 && blockIdx.y == 0) {
+      double v = 0.0;
+      for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi][4];
+      partials[prof.white_partial(t)] = prof.desc.white * v;
+    }
   }
 }
 
-// out[3..6] = 1/2 the tile sums in tile order; 0 when the factorisation failed (out[0] is then -inf already).
+// out[3 .. 3 + NC - 1] = 1/2 the tile sums of the NC partial columns in tile order; 0 when the factorisation failed
+// (out[0] is then -inf already).  NC = 4 for one term, 4 nterms + 1 for a sum.
+template <int NC>
 __global__ void __launch_bounds__(1024)
 grad_finish_kernel(const double* __restrict__ partials, int64_t ntiles, const int32_t* __restrict__ info,
                    double* __restrict__ out) {
-  __shared__ double red[32][4];
-  double s[4] = {0.0, 0.0, 0.0, 0.0};
+  __shared__ double red[32][NC];
+  double s[NC];
+#pragma unroll
+  for (int c = 0; c < NC; ++c) s[c] = 0.0;
   for (int64_t t = threadIdx.x; t < ntiles; t += blockDim.x) {
 #pragma unroll
-    for (int c = 0; c < 4; ++c) s[c] += partials[4 * t + c];
+    for (int c = 0; c < NC; ++c) s[c] += partials[NC * t + c];
   }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
-  for (int c = 0; c < 4; ++c) {
+  for (int c = 0; c < NC; ++c) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) s[c] += __shfl_xor_sync(0xffffffffu, s[c], o);
   }
   if (lane == 0) {
 #pragma unroll
-    for (int c = 0; c < 4; ++c) red[warp][c] = s[c];
+    for (int c = 0; c < NC; ++c) red[warp][c] = s[c];
   }
   __syncthreads();
-  if (threadIdx.x < 4) {
+  if (threadIdx.x < NC) {
     double v = 0.0;
     for (int wi = 0; wi < 32; ++wi) v += red[wi][threadIdx.x];
     out[3 + threadIdx.x] = (*info != 0) ? 0.0 : 0.5 * v;
   }
 }
 
-extern "C" int tgp_loglike_grad(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
-                                double* work, int64_t ld, double* alpha, double* out, int32_t* info,
-                                const int64_t* row_end, int64_t nblocks, double* scratch, void* stream) {
-  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+static int grad_args(const double* X, const double* y, int64_t N, double* work, int64_t ld, const double* alpha,
+                     const double* out, const int32_t* info, const int64_t* row_end, int64_t nblocks,
+                     const double* scratch) {
   TGP_CHECK_ARG(N > 0 && X && y && alpha && out && info, "null pointer / N");
   TGP_CHECK_ARG(!check_args_mat(work, N, ld), "work must be 16-byte aligned with even ld >= N");
   TGP_CHECK_ARG(!check_env(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
   TGP_CHECK_ARG(scratch && ((uintptr_t)scratch & 15) == 0,
                 "scratch: 16-byte aligned buffer of tgp_selinv_work_doubles(N) doubles");
+  TGP_CHECK_ARG(grad_tiles(N) < (1ll << 31), "matrix too large for one launch");
+  return TGP_OK;
+}
+
+// After the likelihood call (alpha = K^-1 y, the factor in `work`): the selected inverse, then the contraction over
+// nterms x tiles CTAs into `ncols` partials per tile, then the finishing kernel.
+template <class P>
+static int grad_tail(const double* X, int64_t N, const P& prof, int nterms, int ncols, double* work, int64_t ld,
+                     const double* alpha, double* out, const int32_t* info, const int64_t* row_end, double* scratch,
+                     cudaStream_t st) {
   const int64_t ntiles = grad_tiles(N);
-  TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
-  cudaStream_t st = (cudaStream_t)stream;
-  int rc = row_end ? tgp_loglike_env(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream)
-                   : tgp_loglike(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, stream);
-  if (rc) return rc;
   const std::vector<int64_t> re = clamped_row_end(row_end, N);
-  rc = selinv_run(work, N, ld, re, scratch, st);
+  int rc = selinv_run(work, N, ld, re, scratch, st);
   if (rc) return rc;
   // the selected-inverse scratch is free again: tile partials at the front, the envelope at the back
   int64_t* re_dev = nullptr;
   if (row_end) {
-    re_dev = reinterpret_cast<int64_t*>(scratch + tgp_selinv_work_doubles(N) - even64((int64_t)re.size()));
+    re_dev = reinterpret_cast<int64_t*>(scratch + grad_work_doubles(N, ncols) - even64((int64_t)re.size()));
     TGP_CUDA(cudaMemcpyAsync(re_dev, re.data(), re.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   }
-  const KDesc kd = make_kdesc(k);
-  const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (grad_contract_kernel<FAM><<<(unsigned)ntiles, GT_THREADS, 0, st>>>(
-                                   X, N, kd, work, ld, alpha, re_dev, scratch, phi)));
+  grad_contract_kernel<P><<<dim3((unsigned)ntiles, (unsigned)nterms), GT_THREADS, 0, st>>>(
+      X, N, prof, work, ld, alpha, re_dev, scratch, tgp_phi_device());
   TGP_LAUNCH_CHECK();
-  grad_finish_kernel<<<1, 1024, 0, st>>>(scratch, ntiles, info, out);
+  switch (ncols) {
+    case 4: grad_finish_kernel<4><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
+    case 5: grad_finish_kernel<5><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
+    case 9: grad_finish_kernel<9><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
+    case 13: grad_finish_kernel<13><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
+    default: grad_finish_kernel<4 * TGP_MAX_TERMS + 1><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
+  }
   TGP_LAUNCH_CHECK();
   return TGP_OK;
+}
+
+extern "C" int tgp_loglike_grad(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
+                                double* work, int64_t ld, double* alpha, double* out, int32_t* info,
+                                const int64_t* row_end, int64_t nblocks, double* scratch, void* stream) {
+  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+  int rc = grad_args(X, y, N, work, ld, alpha, out, info, row_end, nblocks, scratch);
+  if (rc) return rc;
+  rc = row_end ? tgp_loglike_env(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream)
+               : tgp_loglike(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, stream);
+  if (rc) return rc;
+  const KDesc kd = make_kdesc(k);
+  TGP_FAMILY_SWITCH(k->family, return grad_tail(X, N, FamilyProfile<FAM>{kd}, 1, 4, work, ld, alpha, out, info,
+                                                row_end, scratch, (cudaStream_t)stream));
+  return TGP_OK;
+}
+
+extern "C" int tgp_loglike_grad_sum(const double* X, const double* y, const double* yerr2, int64_t N,
+                                    const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, double* out,
+                                    int32_t* info, const int64_t* row_end, int64_t nblocks, double* scratch,
+                                    void* stream) {
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  int rc = grad_args(X, y, N, work, ld, alpha, out, info, row_end, nblocks, scratch);
+  if (rc) return rc;
+  if (k->nterms == 1 && k->white == 0.0) {   // one term: the single-term entry bit for bit, d / d ln white = 0
+    TGP_CUDA(cudaMemsetAsync(out + 7, 0, sizeof(double), (cudaStream_t)stream));
+    return tgp_loglike_grad(X, y, yerr2, N, &k->term[0], work, ld, alpha, out, info, row_end, nblocks, scratch,
+                            stream);
+  }
+  rc = tgp_loglike_sum(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream);
+  if (rc) return rc;
+  return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
+                   row_end, scratch, (cudaStream_t)stream);
 }

@@ -17,7 +17,7 @@ import copy
 import numpy as np
 
 from . import _cabi, backend
-from .kernels import eval_kernel, lower_kernel
+from .kernels import eval_kernel, lower
 from .log_likelihood import log_likelihood
 from .two_pcf import two_pcf
 
@@ -158,7 +158,7 @@ class GPInterpolation(object):
             return
         Xd = backend.as_points(X1)
         n = Xd.shape[0]
-        desc = lower_kernel(kernel, Xd.shape[1])
+        desc = lower(kernel, Xd.shape[1])
         e2 = backend.to_device(np.asarray(y_err, dtype=np.float64).reshape(-1) ** 2)
         yd = backend.to_device(np.asarray(y, dtype=np.float64).reshape(-1))
         # A kernel whose support is short against the field: with the points sorted along one axis K is zero (below
@@ -198,7 +198,7 @@ class GPInterpolation(object):
         y = np.asarray(self._y - self._mean - self._spatial_average, dtype=np.float64).reshape(-1)
         Xd = backend.as_points(self._X)
         n = Xd.shape[0]
-        desc = lower_kernel(self.kernel, Xd.shape[1])
+        desc = lower(self.kernel, Xd.shape[1])
         e2_host = np.asarray(self._y_err, dtype=np.float64).reshape(-1) ** 2
         e2, yd = backend.to_device(e2_host), backend.to_device(y)
         env = backend.plan_envelope(Xd, desc) if self.BANDED_SOLVE else None

@@ -9,7 +9,8 @@ include/treegp_b200.h and runs the tiled CUDA build (csrc/kmat.cu) instead of
 pdist/cdist + scipy.special.kv.
 
 ``lower_kernel`` is the bridge used by GPInterpolation / log_likelihood / two_pcf to keep whole
-solves on the device.
+solves on the device; ``lower_kernel_sum`` lowers sums of such terms plus a ``WhiteKernel`` level, and ``lower``
+picks whichever of the two applies.
 """
 import numpy as np
 from sklearn.gaussian_process import kernels as _skk
@@ -22,13 +23,15 @@ from sklearn.gaussian_process.kernels import (
     Product,
     RBF,
     StationaryKernelMixin,
+    Sum,
+    WhiteKernel,
 )
 
 from . import _cabi
-from ._cabi import TgpKernel
+from ._cabi import TgpKernel, TgpKernelSum
 
 __all__ = ["eval_kernel", "AnisotropicRBF", "VonKarman", "AnisotropicVonKarman", "lower_kernel",
-           "lower_kernel_jacobian"]
+           "lower_kernel_jacobian", "lower_kernel_sum", "lower_kernel_sum_jacobian", "lower", "lower_jacobian"]
 
 
 # ------------------------------------------------------------------------------------------------
@@ -378,3 +381,118 @@ def lower_kernel_jacobian(kernel, ndim):
     if J.shape[1] != len(kernel.theta):
         raise _cabi.TgpError("unsupported kernel for the B200 backend (theta layout): %r" % (kernel,))
     return desc, J
+
+
+# ------------------------------------------------------------------------------------------------
+# sums of stationary terms plus a white-noise level
+# ------------------------------------------------------------------------------------------------
+def _product_factors(k):
+    """Factors of a (nested) Product in theta order."""
+    if isinstance(k, Product):
+        return _product_factors(k.k1) + _product_factors(k.k2)
+    return [k]
+
+
+def _expand_sum(k, ndim):
+    """Distribute the constants of the tree k over its terms.  Returns (terms, whites, cols): terms is a list of
+    TgpKernel (amp included), whites the list of white levels (scale included), and cols one entry per free
+    hyper-parameter of k in theta order: (T, W) with T[c] = d (ln amp_c, m00_c, m01_c, m11_c) / d theta and
+    W[j] = d white_j / d theta."""
+    if isinstance(k, Sum):
+        t1, w1, c1 = _expand_sum(k.k1, ndim)
+        t2, w2, c2 = _expand_sum(k.k2, ndim)
+        pad = [(np.vstack([T, np.zeros((len(t2), 4))]), np.concatenate([W, np.zeros(len(w2))])) for T, W in c1]
+        pad += [(np.vstack([np.zeros((len(t1), 4)), T]), np.concatenate([np.zeros(len(w1)), W])) for T, W in c2]
+        return t1 + t2, w1 + w2, pad
+    if isinstance(k, WhiteKernel):
+        lvl = float(k.noise_level)
+        return [], [lvl], ([] if k.hyperparameter_noise_level.fixed else [(np.zeros((0, 4)), np.array([lvl]))])
+    if isinstance(k, (Product, ConstantKernel)):
+        factors = _product_factors(k)
+        inner = [f for f in factors if not isinstance(f, ConstantKernel)]
+        if len(inner) > 1:
+            raise _cabi.TgpError("unsupported kernel for the B200 backend (more than one non-constant factor): %r"
+                                 % (k,))
+        if not inner:
+            raise _cabi.TgpError("unsupported kernel for the B200 backend (a constant offset term): %r" % (k,))
+        scale = float(np.prod([float(f.constant_value) for f in factors if isinstance(f, ConstantKernel)]))
+        terms, whites, sub = _expand_sum(inner[0], ndim)
+        for t in terms:
+            t.amp *= scale
+        whites = [scale * w for w in whites]
+        cols = []
+        for f in factors:
+            if f is inner[0]:
+                cols += [(T, scale * W) for T, W in sub]
+            elif not f.hyperparameter_constant_value.fixed:   # d ln amp_c / d ln c = 1 for every term under it
+                T = np.zeros((len(terms), 4))
+                T[:, 0] = 1.0
+                cols.append((T, np.array(whites)))
+        return terms, whites, cols
+    desc = lower_kernel(k, ndim)   # raises for anything that is not a supported stationary kernel
+    return [desc], [], [(c[None, :], np.zeros(0)) for c in _factor_jacobian(k, ndim)]
+
+
+def _lower_sum(kernel, ndim):
+    terms, whites, cols = _expand_sum(kernel, ndim)
+    if not terms:
+        raise _cabi.TgpError("unsupported kernel for the B200 backend (no stationary term): %r" % (kernel,))
+    if len(terms) > _cabi.MAX_TERMS:
+        raise _cabi.TgpError("unsupported kernel for the B200 backend (%d stationary terms, at most %d): %r"
+                             % (len(terms), _cabi.MAX_TERMS, kernel))
+    desc = TgpKernelSum()
+    desc.nterms, desc.ndim, desc.white = len(terms), ndim, float(sum(whites))
+    for c, t in enumerate(terms):
+        desc.term[c] = t
+    return desc, whites, cols
+
+
+def lower_kernel_sum(kernel, ndim):
+    """sklearn kernel tree -> ``TgpKernelSum``.
+
+    Accepted: Sum nodes; Products of any number of ``ConstantKernel`` factors and at most one other factor, which may
+    itself be a Sum (the constants distribute over it); leaves are the stationary kernels ``lower_kernel`` accepts and
+    ``WhiteKernel`` (possibly scaled; several add up).  Rejected with ``TgpError``: a product of two non-constant
+    factors, a constant offset term, any other kernel, no stationary term, more than ``TGP_MAX_TERMS`` stationary
+    terms.  Terms keep their order in the tree (k1 before k2)."""
+    return _lower_sum(kernel, ndim)[0]
+
+
+def lower_kernel_sum_jacobian(kernel, ndim):
+    """(``lower_kernel_sum(kernel, ndim)``, J): J is the (4 nterms + 1) x n_theta Jacobian of (ln amp_c, m00_c, m01_c,
+    m11_c for every term c, then ln white) with respect to ``kernel.theta`` -- columns in scikit-learn's theta order
+    (Sum and Product list k1's then k2's), fixed hyper-parameters absent.  The ln white row is 0 when there is no
+    white level.  d logL / d theta = J^T g with g from tgp_loglike_grad_sum."""
+    desc, whites, cols = _lower_sum(kernel, ndim)
+    n, w = desc.nterms, desc.white
+    J = np.zeros((4 * n + 1, len(cols)))
+    for j, (T, W) in enumerate(cols):
+        J[: 4 * n, j] = T.reshape(-1)
+        J[4 * n, j] = float(np.sum(W)) / w if w > 0 else 0.0
+    if J.shape[1] != len(kernel.theta):
+        raise _cabi.TgpError("unsupported kernel for the B200 backend (theta layout): %r" % (kernel,))
+    return desc, J
+
+
+def lower(kernel, ndim):
+    """The device descriptor of a kernel: ``lower_kernel(kernel, ndim)`` whenever it accepts the kernel (every kernel
+    that lowers to one term keeps that path), else ``lower_kernel_sum(kernel, ndim)``."""
+    try:
+        return lower_kernel(kernel, ndim)
+    except _cabi.TgpError:
+        return lower_kernel_sum(kernel, ndim)
+
+
+def lower_jacobian(kernel, ndim):
+    """``lower_kernel_jacobian`` or ``lower_kernel_sum_jacobian``, chosen as ``lower`` chooses."""
+    try:
+        return lower_kernel_jacobian(kernel, ndim)
+    except _cabi.TgpError:
+        return lower_kernel_sum_jacobian(kernel, ndim)
+
+
+def descriptor_params(desc):
+    """Every number of a descriptor (amplitudes, metrics, white level): a non-finite one cannot be factorised."""
+    terms = [desc] if isinstance(desc, TgpKernel) else [desc.term[c] for c in range(desc.nterms)]
+    vals = [v for t in terms for v in (t.amp, t.m00, t.m01, t.m11)]
+    return vals if isinstance(desc, TgpKernel) else vals + [desc.white]

@@ -12,7 +12,7 @@ import numpy as np
 from scipy import optimize
 
 from . import backend
-from .kernels import lower_kernel, lower_kernel_jacobian
+from .kernels import descriptor_params, lower, lower_jacobian
 
 # Multi-GPU (SURVEY.md section 8e): the (n_theta + 1) likelihood evaluations of one forward-difference gradient
 # are independent.  With DISTRIBUTED_FD = True (or env TREEGP_B200_DIST_FD=1) and an initialised process group,
@@ -70,10 +70,10 @@ class log_likelihood(object):
         """log p(y | X, kernel) = -chi2/2 - n/2 ln(2 pi) - ln|K|/2, or -inf when K + diag(y_err^2) is not
         positive definite.  `kernel` is a scikit-learn style kernel object."""
         Xd, yd, e2, work = self._device_state()
-        desc = lower_kernel(kernel, Xd.shape[1])
+        desc = lower(kernel, Xd.shape[1])
         # a non-finite hyper-parameter cannot be factorised: the reference's try/except returns -inf
         # (log_likelihood.py:38-39); same outcome here without launching anything
-        if not np.all(np.isfinite([desc.amp, desc.m00, desc.m01, desc.m11])):
+        if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf
         banded = self._envelope_inputs(desc)
         if banded is None:
@@ -98,8 +98,8 @@ class log_likelihood(object):
         the selected inverse Z = K^-1 inside its envelope and one contraction with alpha alpha^T - Z).  Same envelope
         choice and -inf rule as log_likelihood; the gradient is 0 where the value is -inf."""
         Xd, yd, e2, work = self._device_state()
-        desc, J = lower_kernel_jacobian(kernel, Xd.shape[1])
-        if not np.all(np.isfinite([desc.amp, desc.m00, desc.m01, desc.m11])):
+        desc, J = lower_jacobian(kernel, Xd.shape[1])
+        if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf, np.zeros(J.shape[1])
         banded = self._envelope_inputs(desc)
         if banded is None:
@@ -112,7 +112,7 @@ class log_likelihood(object):
         if o[0] != o[0]:
             from ._cabi import TgpError
             raise TgpError("tgp_loglike_grad: internal synchronisation timed out (info = %d)" % int(info.item()))
-        return float(o[0]), J.T @ o[3:7]
+        return float(o[0]), J.T @ o[3:3 + J.shape[0]]
 
     @staticmethod
     def _value_and_fd_gradient(fun, rank, world):
