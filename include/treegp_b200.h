@@ -203,6 +203,38 @@ int tgp_predict_var_sum(const double* Xs, int64_t M, const double* X, int64_t N,
                         const double* L, int64_t ld, const int64_t* row_end /*host*/, int64_t nblocks, double* work,
                         int64_t chunk, double* var, void* stream);
 
+/* ---- (2e) several outputs sharing one kernel ---------------------------------------------------------------------
+ * r fields measured at the same points with the same errors are r independent GPs with one covariance: K + diag(yerr2)
+ * is built and factorised once for all of them.  Every (N, r) or (M, r) matrix is row-major (numpy's layout);
+ * 1 <= r <= TGP_MAX_RHS.  The kernel is always a tgp_kernel_sum (a single kernel is a one-term sum).  With r == 1
+ * each entry gives bit for bit what its single-output twin gives.  Arguments are checked before any CUDA call. */
+#define TGP_MAX_RHS 8
+/* tgp_loglike_sum for r outputs.  work: (N + r) x ld (r extra rows carry the outputs through the factorisation).
+ * alpha: device double[N * r] = K^-1 Y, or L^-1 Y when want_alpha == 0; each column equals the single-output
+ * alpha of that column bit for bit.  out: device double[3] = {sum_c logL_c, sum_c chi2_c, logdet}, i.e.
+ * logL = -1/2 sum_c y_c^T K^-1 y_c - r/2 ln|K| - r N/2 ln 2 pi; -inf when *info > 0. */
+int tgp_loglike_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
+                      const tgp_kernel_sum* k /*host*/, double* work, int64_t ld, double* alpha, int want_alpha,
+                      double* out, int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, void* stream);
+/* tgp_loglike_grad_sum for r outputs: the gradient of the joint logL, 1/2 tr((sum_c alpha_c alpha_c^T - r K^-1) dK/dp);
+ * d / d ln white = 1/2 white (sum_c |alpha_c|^2 - r tr K^-1).  out has the layout of tgp_loglike_grad_sum.
+ * scratch: 16-byte aligned, tgp_loglike_grad_multi_work_doubles(N, nterms, r) doubles. */
+int64_t tgp_loglike_grad_multi_work_doubles(int64_t N, int32_t nterms, int32_t r);
+/* tgp_potrs_vec for r right-hand sides: B holds r rows of N at pitch ld (the factor's ld), solved in place.  Both
+ * sweeps stream the factor once for all of them; each row equals its own tgp_potrs_vec result bit for bit. */
+int tgp_potrs_multi(const double* L, int64_t N, int64_t ld, double* B, int32_t r, void* stream);
+int tgp_loglike_grad_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
+                           const tgp_kernel_sum* k /*host*/, double* work, int64_t ld, double* alpha, double* out,
+                           int32_t* info, const int64_t* row_end /*host*/, int64_t nblocks, double* scratch,
+                           void* stream);
+/* mean (M, r) = K(Xs, X) alpha (alpha: (N, r)); each pair's profile is evaluated once for all r outputs.  The
+ * truncated form skips what tgp_predict_mean_trunc_sum skips; work: tgp_predict_work_doubles(N) doubles. */
+int tgp_predict_mean_multi(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k /*host*/,
+                           const double* alpha, int32_t r, double* mean, void* stream);
+int tgp_predict_mean_trunc_multi(const double* Xs, int64_t M, const double* X, int64_t N,
+                                 const tgp_kernel_sum* k /*host*/, const double* alpha, int32_t r, double* mean,
+                                 double* work, void* stream);
+
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 
 /* mean[m] = sum_n K(Xs_m, X_n) alpha_n without materialising K(Xs, X).

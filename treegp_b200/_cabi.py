@@ -24,6 +24,7 @@ class TgpKernel(ctypes.Structure):
 
 
 MAX_TERMS = 4   # TGP_MAX_TERMS
+MAX_RHS = 8     # TGP_MAX_RHS: outputs of the multi-output entries
 
 
 class TgpKernelSum(ctypes.Structure):
@@ -68,6 +69,12 @@ SIGNATURES = {
     "tgp_predict_mean_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _vp, _vp, _vp],
     "tgp_predict_var_sum": [_vp, _i64, _vp, _i64, _ksp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
+    "tgp_loglike_multi": [_vp, _vp, _i32, _vp, _i64, _ksp, _vp, _i64, _vp, ctypes.c_int, _vp, _vp, _vp, _i64, _vp],
+    "tgp_loglike_grad_multi_work_doubles": [_i64, _i32, _i32],
+    "tgp_potrs_multi": [_vp, _i64, _i64, _vp, _i32, _vp],
+    "tgp_loglike_grad_multi": [_vp, _vp, _i32, _vp, _i64, _ksp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
+    "tgp_predict_mean_multi": [_vp, _i64, _vp, _i64, _ksp, _vp, _i32, _vp, _vp],
+    "tgp_predict_mean_trunc_multi": [_vp, _i64, _vp, _i64, _ksp, _vp, _i32, _vp, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -100,6 +107,7 @@ SIGNATURES = {
 }
 _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctypes.c_int64,
              "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
+             "tgp_loglike_grad_multi_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 

@@ -183,6 +183,15 @@ def potrs_vec(L, N, b):
     return b
 
 
+def potrs_multi(L, N, B):
+    """Solve L L^T X = B in place for the r rows of B (device tensor (r, >= N) with B.stride(0) == L.stride(0)); one
+    pass over the factor per sweep for all rows (tgp_potrs_multi)."""
+    if B.dim() != 2 or B.stride(0) != L.stride(0) or not 1 <= B.shape[0] <= _cabi.MAX_RHS:
+        raise ValueError("B must be (r, ld) with the factor's row pitch and 1 <= r <= %d" % _cabi.MAX_RHS)
+    check(_cabi.load().tgp_potrs_multi(_p(L), N, L.stride(0), _p(B), int(B.shape[0]), _stream()), "tgp_potrs_multi")
+    return B
+
+
 def trsm_rows(L, N, B, M, row_end=None):
     """B[:M, :N] <- B L^-T in place.  row_end: the factor's envelope (envelope_rows) -- solved blocks are only
     propagated to the rows inside it."""
@@ -291,6 +300,68 @@ def loglike_grad(X, y, yerr2, kdesc, work=None, row_end=None):
     return out, info, alpha, work
 
 
+def as_sum(kdesc):
+    """The descriptor as a TgpKernelSum (the multi-output entries take sums only): a TgpKernel becomes a one-term sum
+    without white, which the device runs with the single-term kernels."""
+    if is_sum(kdesc):
+        return kdesc
+    s = TgpKernelSum()
+    s.nterms, s.ndim, s.white = 1, kdesc.ndim, 0.0
+    s.term[0] = kdesc
+    return s
+
+
+def _multi_args(X, Y, yerr2, work, rows_needed):
+    X = as_points(X)
+    N = X.shape[0]
+    if Y.dim() != 2 or Y.shape[0] != N or not 1 <= Y.shape[1] <= _cabi.MAX_RHS:
+        raise ValueError("Y must have shape (N, r) with 1 <= r <= %d; got %r" % (_cabi.MAX_RHS, tuple(Y.shape)))
+    if yerr2 is not None and tuple(yerr2.shape) != (N,):
+        raise ValueError("yerr2 must have shape (N,) = (%d,); got %r" % (N, tuple(yerr2.shape)))
+    r = int(Y.shape[1])
+    if work is None:
+        work = alloc_matrix(N + r, N, X.device)
+    if work.shape[0] < N + r:
+        raise ValueError("%s workspace needs N+r rows" % rows_needed)
+    return X, N, r, work
+
+
+def loglike_multi(X, Y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
+    """loglike for r outputs sharing the kernel (tgp_loglike_multi): Y (N, r) device tensor.  Returns (out[3] =
+    joint logL, sum of chi2, logdet; info; alpha (N, r); work, N + r rows)."""
+    X, N, r, work = _multi_args(X, Y, yerr2, work, "loglike_multi")
+    Y = Y.contiguous()
+    alpha = torch.empty((N, r), dtype=F64, device=X.device)
+    out = torch.zeros(3, dtype=F64, device=X.device)
+    info = torch.zeros(1, dtype=torch.int32, device=X.device)
+    re = None if row_end is None else _host_i64(row_end)
+    check(_cabi.load().tgp_loglike_multi(_p(X), _p(Y), r, _p(yerr2), N, ctypes.byref(as_sum(kdesc)), _p(work),
+                                         work.stride(0), _p(alpha), int(bool(want_alpha)), _p(out), _p(info), re,
+                                         0 if row_end is None else len(row_end), _stream()), "tgp_loglike_multi")
+    return out, info, alpha, work
+
+
+def loglike_grad_multi(X, Y, yerr2, kdesc, work=None, row_end=None):
+    """loglike_grad for r outputs (tgp_loglike_grad_multi): the joint logL and its gradient, out in the layout of
+    tgp_loglike_grad_sum (4 + 4 nterms entries; a TgpKernel counts as one term).  Returns (out, info, alpha (N, r),
+    work)."""
+    X, N, r, work = _multi_args(X, Y, yerr2, work, "loglike_grad_multi")
+    _check_dims(kdesc, X)
+    Y = Y.contiguous()
+    ks = as_sum(kdesc)
+    lib = _cabi.load()
+    alpha = torch.empty((N, r), dtype=F64, device=X.device)
+    info = torch.zeros(1, dtype=torch.int32, device=X.device)
+    out = torch.zeros(4 + 4 * ks.nterms, dtype=F64, device=X.device)
+    scratch = torch.empty(int(lib.tgp_loglike_grad_multi_work_doubles(int(N), int(ks.nterms), r)), dtype=F64,
+                          device=X.device)
+    re = None if row_end is None else _host_i64(row_end)
+    check(lib.tgp_loglike_grad_multi(_p(X), _p(Y), r, _p(yerr2), N, ctypes.byref(ks), _p(work), work.stride(0),
+                                     _p(alpha), _p(out), _p(info), re, 0 if row_end is None else len(row_end),
+                                     _p(scratch), _stream()), "tgp_loglike_grad_multi")
+    return out, info, alpha, work
+
+
 TRUNC_MIN_M, TRUNC_MIN_N = 16384, 2048   # below this the plain kernel is launch-bound anyway
 
 
@@ -321,6 +392,38 @@ def predict_mean(Xs, X, kdesc, alpha, out=None, truncate=None):
     tmp = torch.empty(M, dtype=F64, device=X.device)
     fn = lib.tgp_predict_mean_trunc_sum if is_sum(kdesc) else lib.tgp_predict_mean_trunc
     check(fn(_p(Xss), M, _p(Xt), N, ctypes.byref(kdesc), _p(at), _p(tmp), _p(work), _stream()), fn.__name__)
+    out[os_] = tmp
+    return out
+
+
+def predict_mean_multi(Xs, X, kdesc, alpha, truncate=None):
+    """predict_mean for r outputs (tgp_predict_mean[_trunc]_multi): alpha (N, r) -> mean (M, r); every pair's
+    profile is evaluated once for all outputs.  Same Hilbert ordering and truncation choice as predict_mean."""
+    Xs, X = as_points(Xs), as_points(X)
+    _check_dims(kdesc, X, Xs)
+    M, N = Xs.shape[0], X.shape[0]
+    if alpha.dim() != 2 or alpha.shape[0] != N or not 1 <= alpha.shape[1] <= _cabi.MAX_RHS:
+        raise ValueError("alpha must have shape (N, r) = (%d, r) with 1 <= r <= %d; got %r"
+                         % (N, _cabi.MAX_RHS, tuple(alpha.shape)))
+    r = int(alpha.shape[1])
+    ks = as_sum(kdesc)
+    lib = _cabi.load()
+    if truncate is None:
+        truncate = M >= TRUNC_MIN_M and N >= TRUNC_MIN_N
+    out = torch.empty((M, r), dtype=F64, device=X.device)
+    if not truncate:
+        check(lib.tgp_predict_mean_multi(_p(Xs), M, _p(X), N, ctypes.byref(ks), _p(alpha.contiguous()), r, _p(out),
+                                         _stream()), "tgp_predict_mean_multi")
+        return out
+    two_d = X.shape[1] == 2
+    zt, zs = torch.zeros(N, dtype=F64, device=X.device), torch.zeros(M, dtype=F64, device=X.device)
+    ot = hilbert_order(X[:, 0].contiguous(), X[:, 1].contiguous() if two_d else zt)
+    os_ = hilbert_order(Xs[:, 0].contiguous(), Xs[:, 1].contiguous() if two_d else zs)
+    Xt, at, Xss = X[ot].contiguous(), alpha[ot].contiguous(), Xs[os_].contiguous()
+    work = torch.empty(int(lib.tgp_predict_work_doubles(N)), dtype=F64, device=X.device)
+    tmp = torch.empty((M, r), dtype=F64, device=X.device)
+    check(lib.tgp_predict_mean_trunc_multi(_p(Xss), M, _p(Xt), N, ctypes.byref(ks), _p(at), r, _p(tmp), _p(work),
+                                           _stream()), "tgp_predict_mean_trunc_multi")
     out[os_] = tmp
     return out
 

@@ -22,6 +22,7 @@
 #include <string.h>
 #include <atomic>
 #include "tgp_common.cuh"
+#include "profile_policy.cuh"
 
 // ============================================================================================
 // gemm_nt_sub
@@ -1255,8 +1256,17 @@ extern "C" int tgp_gemm_nt_sub(double* C, int64_t M, int64_t Nc, int64_t ldc, co
 // Single right-hand-side solves  L w = b  (forward) and  L^T x = w  (backward): persistent sweep kernels in trsv.cu.
 // ============================================================================================
 int tgp_trsv_sweeps(const double* L, int64_t N, int64_t ld, double* b, int which, cudaStream_t st);
+int tgp_trsv_sweeps_multi(const double* L, int64_t N, int64_t ld, double* b, int r, int which, cudaStream_t st);
 static int trsv_backward(const double* L, int64_t N, int64_t ld, double* b, cudaStream_t st) {
   return tgp_trsv_sweeps(L, N, ld, b, 2, st);
+}
+
+extern "C" int tgp_potrs_multi(const double* L, int64_t N, int64_t ld, double* B, int32_t r, void* stream) {
+  TGP_CHECK_ARG(r >= 1 && r <= TGP_MAX_RHS, "number of right-hand sides must be 1 .. TGP_MAX_RHS");
+  TGP_CHECK_ARG(N >= 0 && ld >= N, "N/ld");
+  if (N == 0) return TGP_OK;
+  TGP_CHECK_ARG(L && B, "null pointer");
+  return tgp_trsv_sweeps_multi(L, N, ld, B, r, 3, (cudaStream_t)stream);
 }
 
 extern "C" int tgp_potrs_vec(const double* L, int64_t N, int64_t ld, double* b, void* stream) {
@@ -1425,4 +1435,101 @@ extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* y
   rc = tgp_kmat_sym_sum(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
   if (rc) return rc;
   return loglike_after_build(y, N, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+}
+
+// ============================================================================================
+// Several outputs with one covariance (tgp_loglike_multi): K is built and factorised once; the r outputs ride
+// through the dense factorisation as r extra rows (rows N .. N + r - 1 of `work`, one output per row), and the sweeps
+// stream the factor once for all outputs (tgp_trsv_sweeps_multi), each column in the single-output order, so each
+// column of alpha is the single-output alpha of that column bit for bit.
+// ============================================================================================
+// rows[c][i] = Y[i][c] (to_rows) or Y[i][c] = rows[c][i]
+__global__ void __launch_bounds__(256)
+multi_transpose_kernel(double* __restrict__ Y, int r, double* __restrict__ rows, int64_t ld, int64_t N, int to_rows) {
+  for (int64_t idx = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; idx < N * r;
+       idx += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = idx / r;
+    const int c = (int)(idx - i * r);
+    if (to_rows) rows[c * ld + i] = Y[idx];
+    else Y[idx] = rows[c * ld + i];
+  }
+}
+
+// sum over the 1024 threads in the order of logdet_chi2_kernel; the result is valid in every thread
+__device__ double block_sum_1024(double a, double* s) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  __syncthreads();                                 // s is free
+  if (lane == 0) s[warp] = a;
+  __syncthreads();
+  a = s[lane];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+  return a;
+}
+
+// out = {sum_c logL_c, sum_c chi2_c, logdet}: logdet once; chi2_c = y_c . alpha_c (want_alpha) or |L^-1 y_c|^2,
+// each in the order of the single-output reductions, then added up column by column.  Single CTA of 1024 threads.
+__global__ void __launch_bounds__(1024)
+loglike_multi_finish_kernel(const double* __restrict__ L, int64_t N, int64_t ld, const double* __restrict__ Y, int r,
+                            const double* __restrict__ W, int want_alpha, const int32_t* __restrict__ info,
+                            double* __restrict__ out) {
+  __shared__ double s[32];
+  double a = 0.0;
+  for (int64_t i = threadIdx.x; i < N; i += blockDim.x) a += 2.0 * log(L[i * ld + i]);
+  const double logdet = block_sum_1024(a, s);
+  double chi2 = 0.0;
+  for (int c = 0; c < r; ++c) {
+    const double* w = W + c * ld;
+    double v = 0.0;
+    for (int64_t i = threadIdx.x; i < N; i += blockDim.x) v = want_alpha ? fma(Y[i * r + c], w[i], v) : fma(w[i], w[i], v);
+    chi2 += block_sum_1024(v, s);
+  }
+  if (threadIdx.x == 0) {
+    double ll = -0.5 * chi2 - 0.5 * (double)r * (double)N * log(2.0 * TGP_PI) - 0.5 * (double)r * logdet;
+    if (*info > 0 || isnan(ll)) ll = -INFINITY;   // as loglike_finish_kernel
+    if (*info < 0) ll = NAN;
+    out[0] = ll;
+    out[1] = chi2;
+    out[2] = logdet;
+  }
+}
+
+extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
+                                 const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
+                                 double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
+  TGP_CHECK_ARG(r >= 1 && r <= TGP_MAX_RHS, "number of outputs must be 1 .. TGP_MAX_RHS");
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  int rc = loglike_args(X, Y, N, work, alpha, out, info, row_end, nblocks);
+  if (rc) return rc;
+  TGP_CHECK_ARG(!check_mat(work, N, ld), "work must be 16-byte aligned with even ld >= N");
+  if (r == 1)   // (N, 1) is an N-vector: the single-output entry, bit for bit
+    return tgp_loglike_sum(X, Y, yerr2, N, k, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+  cudaStream_t st = (cudaStream_t)stream;
+  rc = tgp_kmat_sym_sum(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
+  if (rc) return rc;
+  double* rows = work + N * ld;                    // output c in row N + c
+  const unsigned tg = (unsigned)tgp_cdiv(N * r, (int64_t)256) < 4096u ? (unsigned)tgp_cdiv(N * r, (int64_t)256) : 4096u;
+  multi_transpose_kernel<<<tg, 256, 0, st>>>(const_cast<double*>(Y), r, rows, ld, N, 1);
+  TGP_LAUNCH_CHECK();
+  if (row_end) {
+    // as loglike_after_build: the envelope factorisation, then both sweeps per output
+    rc = tgp_potrf_env(work, N, ld, row_end, nblocks, 0, info, stream);
+    if (rc) return rc;
+    rc = tgp_trsv_sweeps_multi(work, N, ld, rows, r, want_alpha ? 3 : 1, st);
+    if (rc) return rc;
+  } else {
+    rc = tgp_potrf_rows(work, N, ld, r, info, stream);   // rows <- L^-1 Y^T
+    if (rc) return rc;
+    if (want_alpha) {
+      rc = tgp_trsv_sweeps_multi(work, N, ld, rows, r, 2, st);
+      if (rc) return rc;
+    }
+  }
+  loglike_multi_finish_kernel<<<1, 1024, 0, st>>>(work, N, ld, Y, r, rows, want_alpha, info, out);
+  TGP_LAUNCH_CHECK();
+  multi_transpose_kernel<<<tg, 256, 0, st>>>(alpha, r, rows, ld, N, 0);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
 }

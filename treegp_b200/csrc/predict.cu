@@ -13,13 +13,18 @@ constexpr int PM_TILE = 1024;     // training points per shared-memory tile
 // grid: (ceil(M / PM_THREADS), nsplit).  Split s handles training tiles s, s + nsplit, ...
 // nsplit == 1 writes mean directly; otherwise partial sums are added with red.global.add.f64 into a
 // zeroed output (used only when M alone cannot fill the machine).
+// Several outputs (P = MultiOut<..., R>): alpha and mean are row-major (N, r) and (M, r); each thread keeps R pairs of
+// accumulators, evaluates every pair's profile once and applies it to all columns -- each column in the order of the
+// single-output kernel.  The tile shrinks with R so that the staged alpha stays at 16 KB.
 template <class P>
 __global__ void __launch_bounds__(PM_THREADS)
 predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
                     P prof, const double* __restrict__ alpha, double* __restrict__ mean,
                     const double* __restrict__ phi_g) {
-  __shared__ double2 pxy[PM_TILE];
-  __shared__ double pa[PM_TILE];
+  constexpr int R = OutputsOf<P>::kR;
+  constexpr int TILE = R == 1 ? PM_TILE : 2048 / R;
+  __shared__ double2 pxy[TILE];
+  __shared__ double pa[TILE * R];
   __shared__ double phi_s[P::kPhiSize];
   const int tid = threadIdx.x;
   if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
@@ -28,22 +33,32 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
   const double sx = live ? Xs[m * prof.desc.ndim] : 0.0;
   const double sy = (live && prof.desc.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
   const int nsplit = gridDim.y;
-  const int64_t ntile = (N + PM_TILE - 1) / PM_TILE;
+  const int64_t ntile = (N + TILE - 1) / TILE;
   double acc0 = 0.0, acc1 = 0.0;
+  double accm0[R], accm1[R];
+#pragma unroll
+  for (int c = 0; c < R; ++c) accm0[c] = accm1[c] = 0.0;
   for (int64_t tl = blockIdx.y; tl < ntile; tl += nsplit) {
-    const int64_t n0 = tl * PM_TILE;
+    const int64_t n0 = tl * TILE;
     __syncthreads();
-    for (int i = tid; i < PM_TILE; i += PM_THREADS) {
+    for (int i = tid; i < TILE; i += PM_THREADS) {
       const int64_t n = n0 + i;
       const bool ok = n < N;
       double2 p;
       p.x = ok ? X[n * prof.desc.ndim] : 0.0;
       p.y = (ok && prof.desc.ndim == 2) ? X[n * 2 + 1] : 0.0;
       pxy[i] = p;
-      pa[i] = ok ? prof.weight() * alpha[n] : 0.0;  // padded points carry zero weight
+      if constexpr (R == 1) {
+        pa[i] = ok ? prof.weight() * alpha[n] : 0.0;  // padded points carry zero weight
+      } else {
+#pragma unroll
+        for (int c = 0; c < R; ++c) pa[i * R + c] = (ok && c < prof.nrhs) ? prof.weight() * alpha[n * prof.nrhs + c] : 0.0;
+      }
     }
     __syncthreads();
-    if constexpr (P::kSum) {
+    if constexpr (R > 1) {
+      for (int i = 0; i < TILE; i += 2) prof.mean2_multi(sx, sy, pxy, pa, i, phi_s, accm0, accm1);
+    } else if constexpr (P::kSum) {
       for (int i = 0; i < PM_TILE; i += 2) prof.mean2(sx, sy, pxy, pa, i, phi_s, acc0, acc1);
     } else {
       const KDesc& kd = prof.desc;
@@ -58,9 +73,20 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
     }
   }
   if (live) {
-    const double v = acc0 + acc1;
-    if (nsplit == 1) mean[m] = v;
-    else atomicAdd(mean + m, v);
+    if constexpr (R == 1) {
+      const double v = acc0 + acc1;
+      if (nsplit == 1) mean[m] = v;
+      else atomicAdd(mean + m, v);
+    } else {
+#pragma unroll
+      for (int c = 0; c < R; ++c) {
+        if (c < prof.nrhs) {
+          const double v = accm0[c] + accm1[c];
+          if (nsplit == 1) mean[m * prof.nrhs + c] = v;
+          else atomicAdd(mean + m * prof.nrhs + c, v);
+        }
+      }
+    }
   }
 }
 
@@ -72,13 +98,16 @@ static int predict_mean_launch(const double* Xs, int64_t M, const double* X, int
   TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha)), "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t gx = tgp_cdiv(M, PM_THREADS);
-  const int64_t ntile = tgp_cdiv(N, PM_TILE);
+  constexpr int R = OutputsOf<P>::kR;
+  int64_t nout = 1;
+  if constexpr (R > 1) nout = prof.nrhs;
+  const int64_t ntile = tgp_cdiv(N, (int64_t)(R == 1 ? PM_TILE : 2048 / R));
   int64_t nsplit = 1;
   const int64_t target = 4ll * tgp_num_sms();
   if (gx < target) nsplit = tgp_cdiv(target, gx);
   if (nsplit > ntile) nsplit = ntile > 0 ? ntile : 1;
   if (nsplit > 65535) nsplit = 65535;
-  if (nsplit > 1 || N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * sizeof(double), st));
+  if (nsplit > 1 || N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * nout * sizeof(double), st));
   if (N == 0) return TGP_OK;
   dim3 grid((unsigned)gx, (unsigned)nsplit);
   predict_mean_kernel<P><<<grid, PM_THREADS, 0, st>>>(Xs, M, X, N, prof, alpha, mean, tgp_phi_device());
@@ -155,13 +184,14 @@ point_boxes_kernel(const double* __restrict__ X, int64_t N, int ndim, double* __
 }
 
 template <class P>
-__global__ void __launch_bounds__(PM_THREADS)
+__global__ void __launch_bounds__(PM_THREADS, OutputsOf<P>::kR > 1 ? 1 : 0)
 predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
                           P prof, const double* __restrict__ alpha, double* __restrict__ mean,
                           const double* __restrict__ phi_g, const double* __restrict__ boxes, int64_t ngroups,
                           double r2cut) {
+  constexpr int R = OutputsOf<P>::kR;
   __shared__ double2 pxy[PG];
-  __shared__ double pa[PG];
+  __shared__ double pa[PG * R];
   __shared__ double phi_s[P::kPhiSize];
   __shared__ double red[8][4];
   __shared__ int list[PM_THREADS];
@@ -189,6 +219,9 @@ predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double
     by0 = fmin(by0, red[w][2]); by1 = fmax(by1, red[w][3]);
   }
   double acc0 = 0.0, acc1 = 0.0;
+  double accm0[R], accm1[R];
+#pragma unroll
+  for (int c = 0; c < R; ++c) accm0[c] = accm1[c] = 0.0;
   for (int64_t g0 = 0; g0 < ngroups; g0 += PM_THREADS) {
     // which of the next 256 groups can hold a point within the cut-off of any of our test points?
     const int64_t g = g0 + tid;
@@ -221,10 +254,18 @@ predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double
         p.x = ok ? X[n * prof.desc.ndim] : 0.0;
         p.y = (ok && prof.desc.ndim == 2) ? X[n * 2 + 1] : 0.0;
         pxy[tid] = p;
-        pa[tid] = ok ? prof.weight() * alpha[n] : 0.0;
+        if constexpr (R == 1) {
+          pa[tid] = ok ? prof.weight() * alpha[n] : 0.0;
+        } else {
+#pragma unroll
+          for (int c = 0; c < R; ++c)
+            pa[tid * R + c] = (ok && c < prof.nrhs) ? prof.weight() * alpha[n * prof.nrhs + c] : 0.0;
+        }
       }
       __syncthreads();
-      if constexpr (P::kSum) {
+      if constexpr (R > 1) {
+        for (int i = 0; i < PG; i += 2) prof.mean2_multi(sx, sy, pxy, pa, i, phi_s, accm0, accm1);
+      } else if constexpr (P::kSum) {
         for (int i = 0; i < PG; i += 2) prof.mean2(sx, sy, pxy, pa, i, phi_s, acc0, acc1);
       } else {
 #pragma unroll 2
@@ -238,7 +279,13 @@ predict_mean_trunc_kernel(const double* __restrict__ Xs, int64_t M, const double
       }
     }
   }
-  if (live) mean[m] = acc0 + acc1;
+  if constexpr (R == 1) {
+    if (live) mean[m] = acc0 + acc1;
+  } else {
+#pragma unroll
+    for (int c = 0; c < R; ++c)
+      if (live && c < prof.nrhs) mean[m * prof.nrhs + c] = accm0[c] + accm1[c];
+  }
 }
 
 // smallest eigenvalue of the inverse metric: q >= lmin |delta|^2
@@ -310,6 +357,69 @@ extern "C" int tgp_predict_mean_trunc_sum(const double* Xs, int64_t M, const dou
     if (r2 > r2cut) r2cut = r2;
   }
   return predict_mean_trunc_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r2cut, alpha, mean, work, stream);
+}
+
+// ---- several outputs ----------------------------------------------------------------------------------------------
+// r is padded to R = 2, 4 or 8 accumulator columns; a one-term sum without white uses the single-term profile.
+template <int R, class Q>
+static int mean_multi_launch_r(const double* Xs, int64_t M, const double* X, int64_t N, const Q& prof, int r,
+                               double r2cut, const double* alpha, double* mean, double* work, void* stream) {
+  const MultiOut<Q, R> mp{prof, r};
+  if (work) return predict_mean_trunc_launch(Xs, M, X, N, mp, r2cut, alpha, mean, work, stream);
+  return predict_mean_launch(Xs, M, X, N, mp, alpha, mean, stream);
+}
+
+template <class Q>
+static int mean_multi_launch(const double* Xs, int64_t M, const double* X, int64_t N, const Q& prof, int r,
+                             double r2cut, const double* alpha, double* mean, double* work, void* stream) {
+  if (r <= 2) return mean_multi_launch_r<2>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
+  if (r <= 4) return mean_multi_launch_r<4>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
+  return mean_multi_launch_r<8>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
+}
+
+// work == nullptr: the full sum; otherwise the truncated one with the cut-off of tgp_predict_mean_trunc_sum
+static int predict_mean_multi_impl(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
+                                   const double* alpha, int r, double* mean, double* work, void* stream) {
+  TGP_CHECK_ARG(r >= 1 && r <= TGP_MAX_RHS, "number of outputs must be 1 .. TGP_MAX_RHS");
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  if (r == 1)   // (N, 1) and (M, 1) are vectors: the single-output entries, bit for bit
+    return work ? tgp_predict_mean_trunc_sum(Xs, M, X, N, k, alpha, mean, work, stream)
+                : tgp_predict_mean_sum(Xs, M, X, N, k, alpha, mean, stream);
+  TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
+  if (M == 0) return TGP_OK;
+  TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha)), "null pointer");
+  if (N == 0) {
+    TGP_CUDA(cudaMemsetAsync(mean, 0, M * r * sizeof(double), (cudaStream_t)stream));
+    return TGP_OK;
+  }
+  double r2cut = 0.0;
+  if (work) {
+    for (int c = 0; c < k->nterms; ++c) {
+      const double lmin = metric_lmin(&k->term[c]);
+      TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
+      const double r2 = profile_qcut(k->term[c].family) / lmin;
+      if (r2 > r2cut) r2cut = r2;
+    }
+  }
+  if (k->nterms == 1) {
+    const KDesc kd = make_kdesc(&k->term[0]);
+    TGP_FAMILY_SWITCH(k->term[0].family, return mean_multi_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, r, r2cut, alpha,
+                                                                  mean, work, stream));
+    return TGP_OK;
+  }
+  return mean_multi_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r, r2cut, alpha, mean, work, stream);
+}
+
+extern "C" int tgp_predict_mean_multi(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
+                                      const double* alpha, int32_t r, double* mean, void* stream) {
+  return predict_mean_multi_impl(Xs, M, X, N, k, alpha, r, mean, nullptr, stream);
+}
+
+extern "C" int tgp_predict_mean_trunc_multi(const double* Xs, int64_t M, const double* X, int64_t N,
+                                            const tgp_kernel_sum* k, const double* alpha, int32_t r, double* mean,
+                                            double* work, void* stream) {
+  TGP_CHECK_ARG(work != nullptr || M == 0 || N == 0, "work");
+  return predict_mean_multi_impl(Xs, M, X, N, k, alpha, r, mean, work, stream);
 }
 
 // var[m] = amp - sum_n V[m][n]^2, V = K(Xs, X) L^-T (row m = L^-1 k*_m).  Warp per row.

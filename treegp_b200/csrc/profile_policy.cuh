@@ -36,6 +36,21 @@ static inline KSumDesc make_ksumdesc(const tgp_kernel_sum* ks) {
   return d;
 }
 
+// Several outputs sharing one kernel: the policy P with nrhs = r columns of alpha (row-major (N, r)), padded to R
+// columns where a kernel keeps them in registers or shared memory.  OutputsOf<P>::kR is 1 for a plain policy.
+template <class P, int R>
+struct MultiOut : P {
+  int nrhs;
+};
+template <class P>
+struct OutputsOf {
+  static constexpr int kR = 1;
+};
+template <class P, int R>
+struct OutputsOf<MultiOut<P, R>> {
+  static constexpr int kR = R;
+};
+
 #ifdef __CUDACC__
 __device__ __forceinline__ double tgp_profile_rt(int family, double q, const double* __restrict__ phi) {
   switch (family) {
@@ -78,6 +93,20 @@ struct FamilyProfile {
                                          const double* phi_s, double& v0, double& v1) const {
     v0 = desc.amp * tgp_profile<FAM>(tgp_qform(desc, rx - cx0, ry - cy0), phi_s);
     v1 = desc.amp * tgp_profile<FAM>(tgp_qform(desc, rx - cx1, ry - cy1), phi_s);
+  }
+
+  // several outputs: acc[c] += f(q) pa[., c] for training points i, i + 1 of the staged tile (pa: R columns per point)
+  template <int R>
+  __device__ __forceinline__ void mean2_multi(double sx, double sy, const double2* pxy, const double* pa, int i,
+                                              const double* phi_s, double (&acc0)[R], double (&acc1)[R]) const {
+    const double2 p0 = pxy[i], p1 = pxy[i + 1];
+    const double f0 = tgp_profile<FAM>(tgp_qform(desc, sx - p0.x, sy - p0.y), phi_s);
+    const double f1 = tgp_profile<FAM>(tgp_qform(desc, sx - p1.x, sy - p1.y), phi_s);
+#pragma unroll
+    for (int c = 0; c < R; ++c) {
+      acc0[c] = fma(f0, pa[i * R + c], acc0[c]);
+      acc1[c] = fma(f1, pa[(i + 1) * R + c], acc1[c]);
+    }
   }
 
   // gradient contraction: the term a CTA works on, its f, f' and the von Karman rule
@@ -145,6 +174,24 @@ struct SumProfile {
       const KDesc& kd = desc.term[c];
       acc0 = fma(tgp_profile_rt(kd.family, tgp_qform(kd, sx - p0.x, sy - p0.y), phi_s), kd.amp * a0, acc0);
       acc1 = fma(tgp_profile_rt(kd.family, tgp_qform(kd, sx - p1.x, sy - p1.y), phi_s), kd.amp * a1, acc1);
+    }
+  }
+
+  // mean2 for R outputs: each term's profile once per pair, applied to every column (pa: R columns per point)
+  template <int R>
+  __device__ __forceinline__ void mean2_multi(double sx, double sy, const double2* pxy, const double* pa, int i,
+                                              const double* phi_s, double (&acc0)[R], double (&acc1)[R]) const {
+    const double2 p0 = pxy[i], p1 = pxy[i + 1];
+#pragma unroll 1
+    for (int c = 0; c < desc.nterms; ++c) {
+      const KDesc& kd = desc.term[c];
+      const double f0 = tgp_profile_rt(kd.family, tgp_qform(kd, sx - p0.x, sy - p0.y), phi_s);
+      const double f1 = tgp_profile_rt(kd.family, tgp_qform(kd, sx - p1.x, sy - p1.y), phi_s);
+#pragma unroll
+      for (int j = 0; j < R; ++j) {
+        acc0[j] = fma(f0, kd.amp * pa[i * R + j], acc0[j]);
+        acc1[j] = fma(f1, kd.amp * pa[(i + 1) * R + j], acc1[j]);
+      }
     }
   }
 

@@ -34,6 +34,9 @@ extern "C" int tgp_envelope_block(void);
 extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N,
                                const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
                                double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream);
+extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
+                                 const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
+                                 double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream);
 
 constexpr int SB = 512;            // block columns of the recurrence: the envelope's block (tgp_envelope_block)
 constexpr int GT = 64;             // contraction tile edge
@@ -58,6 +61,12 @@ extern "C" int64_t tgp_selinv_work_doubles(int64_t N) { return grad_work_doubles
 extern "C" int64_t tgp_loglike_grad_sum_work_doubles(int64_t N, int32_t nterms) {
   if (nterms < 1 || nterms > TGP_MAX_TERMS) return -1;
   return grad_work_doubles(N, 4 * nterms + 1);
+}
+
+// the outputs change the contraction's weights, not its partial sums
+extern "C" int64_t tgp_loglike_grad_multi_work_doubles(int64_t N, int32_t nterms, int32_t r) {
+  if (r < 1 || r > TGP_MAX_RHS) return -1;
+  return tgp_loglike_grad_sum_work_doubles(N, nterms);
 }
 
 // ---- small helpers --------------------------------------------------------------------------------------------
@@ -201,12 +210,15 @@ extern "C" int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_e
 // Sums (SumProfile): CTA (t, c) contracts term c of tile t into columns 4 c .. 4 c + 3 of the tile's 4 nterms + 1
 // partials; the CTAs of term 0 also sum w_ii = alpha_i^2 - Z_ii over the diagonal, times the white level, into the
 // last column (d K / d ln white = white I).
+//
+// Several outputs (P = MultiOut<..., TGP_MAX_RHS>, nrhs = r columns of alpha): w_ij = sum_c alpha_ic alpha_jc - r Z_ij.
 template <class P>
 __global__ void __launch_bounds__(GT_THREADS)
 grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ Z, int64_t ld,
                      const double* __restrict__ alpha, const int64_t* __restrict__ re_dev,
                      double* __restrict__ partials, const double* __restrict__ phi_g) {
-  __shared__ double xr[GT], yr[GT], ar[GT], xc[GT], yc[GT], ac[GT];
+  constexpr int RM = OutputsOf<P>::kR;
+  __shared__ double xr[GT], yr[GT], ar[GT * RM], xc[GT], yc[GT], ac[GT * RM];
   __shared__ double red[GT_THREADS / 32][P::kSum ? 5 : 4];
   __shared__ double phi_s[P::kPhiSize];
   const KDesc& kd = prof.grad_term();
@@ -231,14 +243,22 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const doub
     const bool ok = r < N;
     xr[tid] = ok ? X[r * kd.ndim] : 0.0;
     yr[tid] = (ok && kd.ndim == 2) ? X[r * 2 + 1] : 0.0;
-    ar[tid] = ok ? alpha[r] : 0.0;
+    if constexpr (RM > 1) {
+      for (int c = 0; c < prof.nrhs; ++c) ar[tid * RM + c] = ok ? alpha[r * prof.nrhs + c] : 0.0;
+    } else {
+      ar[tid] = ok ? alpha[r] : 0.0;
+    }
   } else if (tid < 2 * GT) {
     const int l = tid - GT;
     const int64_t c = c0 + l;
     const bool ok = c < N;
     xc[l] = ok ? X[c * kd.ndim] : 0.0;
     yc[l] = (ok && kd.ndim == 2) ? X[c * 2 + 1] : 0.0;
-    ac[l] = ok ? alpha[c] : 0.0;
+    if constexpr (RM > 1) {
+      for (int j = 0; j < prof.nrhs; ++j) ac[l * RM + j] = ok ? alpha[c * prof.nrhs + j] : 0.0;
+    } else {
+      ac[l] = ok ? alpha[c] : 0.0;
+    }
   }
   __syncthreads();
   const int lane = tid & 31, warp = tid >> 5;
@@ -256,7 +276,16 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const doub
       if (cg > rg) continue;
       const double dx = xr[rl] - xc[cl], dy = yr[rl] - yc[cl];
       const double q = tgp_qform(kd, dx, dy);
-      const double wij = (rg == cg ? 1.0 : 2.0) * (ar[rl] * ac[cl] - Z[rg * ld + cg]);
+      double wij;
+      if constexpr (RM > 1) {
+        const double* a = ar + rl * RM;
+        const double* b = ac + cl * RM;
+        double aa = a[0] * b[0];
+        for (int c = 1; c < prof.nrhs; ++c) aa = fma(a[c], b[c], aa);
+        wij = (rg == cg ? 1.0 : 2.0) * (aa - (double)prof.nrhs * Z[rg * ld + cg]);
+      } else {
+        wij = (rg == cg ? 1.0 : 2.0) * (ar[rl] * ac[cl] - Z[rg * ld + cg]);
+      }
       double f = prof.f(kd, q, phi_s);
       // K(X, X) of the von Karman kernels is 0 between distinct coincident points (kmat.cu, kernels.py:253-262)
       if (prof.vk(kd) && q == 0.0 && rg != cg) f = 0.0;
@@ -350,7 +379,7 @@ static int grad_args(const double* X, const double* y, int64_t N, double* work, 
 template <class P>
 static int grad_tail(const double* X, int64_t N, const P& prof, int nterms, int ncols, double* work, int64_t ld,
                      const double* alpha, double* out, const int32_t* info, const int64_t* row_end, double* scratch,
-                     cudaStream_t st) {
+                     cudaStream_t st, int nrhs = 1) {
   const int64_t ntiles = grad_tiles(N);
   const std::vector<int64_t> re = clamped_row_end(row_end, N);
   int rc = selinv_run(work, N, ld, re, scratch, st);
@@ -361,8 +390,13 @@ static int grad_tail(const double* X, int64_t N, const P& prof, int nterms, int 
     re_dev = reinterpret_cast<int64_t*>(scratch + grad_work_doubles(N, ncols) - even64((int64_t)re.size()));
     TGP_CUDA(cudaMemcpyAsync(re_dev, re.data(), re.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
   }
-  grad_contract_kernel<P><<<dim3((unsigned)ntiles, (unsigned)nterms), GT_THREADS, 0, st>>>(
-      X, N, prof, work, ld, alpha, re_dev, scratch, tgp_phi_device());
+  if (nrhs == 1) {
+    grad_contract_kernel<P><<<dim3((unsigned)ntiles, (unsigned)nterms), GT_THREADS, 0, st>>>(
+        X, N, prof, work, ld, alpha, re_dev, scratch, tgp_phi_device());
+  } else {
+    grad_contract_kernel<MultiOut<P, TGP_MAX_RHS>><<<dim3((unsigned)ntiles, (unsigned)nterms), GT_THREADS, 0, st>>>(
+        X, N, MultiOut<P, TGP_MAX_RHS>{prof, nrhs}, work, ld, alpha, re_dev, scratch, tgp_phi_device());
+  }
   TGP_LAUNCH_CHECK();
   switch (ncols) {
     case 4: grad_finish_kernel<4><<<1, 1024, 0, st>>>(scratch, ntiles, info, out); break;
@@ -406,4 +440,28 @@ extern "C" int tgp_loglike_grad_sum(const double* X, const double* y, const doub
   if (rc) return rc;
   return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
                    row_end, scratch, (cudaStream_t)stream);
+}
+
+extern "C" int tgp_loglike_grad_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
+                                      const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, double* out,
+                                      int32_t* info, const int64_t* row_end, int64_t nblocks, double* scratch,
+                                      void* stream) {
+  TGP_CHECK_ARG(r >= 1 && r <= TGP_MAX_RHS, "number of outputs must be 1 .. TGP_MAX_RHS");
+  TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
+  int rc = grad_args(X, Y, N, work, ld, alpha, out, info, row_end, nblocks, scratch);
+  if (rc) return rc;
+  if (r == 1)   // (N, 1) is an N-vector: the single-output entry, bit for bit
+    return tgp_loglike_grad_sum(X, Y, yerr2, N, k, work, ld, alpha, out, info, row_end, nblocks, scratch, stream);
+  rc = tgp_loglike_multi(X, Y, r, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream);
+  if (rc) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (k->nterms == 1 && k->white == 0.0) {   // one term: the single-term contraction, d / d ln white = 0
+    TGP_CUDA(cudaMemsetAsync(out + 7, 0, sizeof(double), st));
+    const KDesc kd = make_kdesc(&k->term[0]);
+    TGP_FAMILY_SWITCH(k->term[0].family, return grad_tail(X, N, FamilyProfile<FAM>{kd}, 1, 4, work, ld, alpha, out,
+                                                          info, row_end, scratch, st, r));
+    return TGP_OK;
+  }
+  return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
+                   row_end, scratch, st, r);
 }

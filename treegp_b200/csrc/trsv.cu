@@ -245,17 +245,21 @@ __device__ __forceinline__ double2 ldg2(const double* p, bool vec) {
   return make_double2(__ldcs(p), __ldcs(p + 1));
 }
 
-template <bool FWD>
+// R right-hand sides (columns b + c ld, c < R) in one sweep: the factor is streamed once for all of them.  Everything
+// that holds unknowns gets R columns of 64 -- a window block [g][c][64], a published block [c][64], acc [slab][c][64]
+// (backward [slab][warp][c][64]) -- and every column is accumulated and solved in the order of the R = 1 sweep, so each
+// column equals its own single right-hand-side run bit for bit when the grid is the same.
+template <bool FWD, int R>
 __global__ void __launch_bounds__(TS_THREADS, 1)
 trsv_sweep_kernel(TrsvParams P) {
   extern __shared__ __align__(128) unsigned char smraw[];
   double* dtile = reinterpret_cast<double*>(smraw);                // D_k of the next chain step
   double* wtile = dtile + TS_TILE_D;                               // W_k / M_k of the next chain step
   double* xs = wtile + TS_TILE_D;                                  // window of unknowns: TS_WIN column blocks
-  double* xh = xs + TS_WIN * TS;                                   // hand-over buffers [slab parity][distance 1..TS_HAND][64]:
-  double* vs = xh + 2 * TS_HAND * TS;                              // unknowns of the TS_NEAR blocks before a slab's diagonal; vs = b_k - partial sums
-  double* bs = vs + TS;                                            // b of the next chain step (prefetched)
-  double* red = bs + TS;                                           // 4 x 64 partials (backward chain step)
+  double* xh = xs + TS_WIN * TS * R;                               // hand-over buffers [slab parity][distance 1..TS_HAND][64]:
+  double* vs = xh + 2 * TS_HAND * TS * R;                          // unknowns of the TS_NEAR blocks before a slab's diagonal; vs = b_k - partial sums
+  double* bs = vs + TS * R;                                        // b of the next chain step (prefetched)
+  double* red = bs + TS * R;                                       // 4 x 64 partials (backward chain step)
   uint64_t* full = reinterpret_cast<uint64_t*>(red + 4 * TS);      // [0] D/W tiles landed, [1] xc filled by a cluster peer
   double* acc = reinterpret_cast<double*>(full + 2);               // forward [slab][64]; backward [slab][warp][64]
 
@@ -265,7 +269,7 @@ trsv_sweep_kernel(TrsvParams P) {
   const int64_t ld = P.ld, N = P.N;
   const bool vec = P.aligned != 0;
   const int CS = P.CS;
-  constexpr int ACC_PER_SLAB = FWD ? TS : 8 * TS;
+  constexpr int ACC_PER_SLAB = (FWD ? TS : 8 * TS) * R;
 
   // primed block index -> first row / column of the block in the matrix, and its height
   auto blk0 = [&](int kp) -> int64_t { return (int64_t)(FWD ? kp : nb - 1 - kp) * TS; };
@@ -276,7 +280,7 @@ trsv_sweep_kernel(TrsvParams P) {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   for (int i = tid; i < M * ACC_PER_SLAB; i += TS_THREADS) acc[i] = 0.0;
-  for (int i = tid; i < 2 * TS_HAND * TS; i += TS_THREADS) xh[i] = __longlong_as_double(-1ll);   // "nothing handed over yet"
+  for (int i = tid; i < 2 * TS_HAND * TS * R; i += TS_THREADS) xh[i] = __longlong_as_double(-1ll);   // "nothing handed over yet"
   __syncthreads();
   if (CS > 1) cluster_sync_all();                  // every peer's xc is initialised before anyone stores into it
   // The owner of slab k + 1 is CTA (c + 1) mod G, that of slab k - 1 CTA (c - 1) mod G: inside one cluster the
@@ -302,7 +306,12 @@ trsv_sweep_kernel(TrsvParams P) {
     if (tid < TS) {
       bulk_g2s(dtile + tid * TS_P, P.dinv + blk + tid * TS, TS * 8, &full[0]);
       if (kp >= 1) bulk_g2s(wtile + tid * TS_P, P.wmat + blk + tid * TS, TS * 8, &full[0]);
-      bs[tid] = (tid < w) ? P.b[r0 + tid] : 0.0;
+      if constexpr (R == 1) {
+        bs[tid] = (tid < w) ? P.b[r0 + tid] : 0.0;
+      } else {
+#pragma unroll
+        for (int c = 0; c < R; ++c) bs[c * TS + tid] = (tid < w) ? P.b[c * P.ld + r0 + tid] : 0.0;
+      }
     }
   };
 
@@ -357,65 +366,136 @@ trsv_sweep_kernel(TrsvParams P) {
     const int64_t r0 = blk0(kp);
     const int w = blkw(kp);
     __syncthreads();                               // every warp has booked its part of acc
-    if (owner) {
-      double a;
-      if (FWD) {
-        a = acc[ms * TS + idx];
-      } else {                                     // the eight warps' partial sums, in a fixed order
-        const double* p = acc + ms * 8 * TS + idx;
-        a = ((p[0] + p[TS]) + (p[2 * TS] + p[3 * TS])) + ((p[4 * TS] + p[5 * TS]) + (p[6 * TS] + p[7 * TS]));
-      }
-      vs[idx] = (idx < w) ? bs[idx] - a : 0.0;
-    }
-    mbar_wait(&full[0], dphase);
-    dphase ^= 1;
-    __syncthreads();
-    double xv = matvec(dtile, vs, TS);
-    double* xc = xh + ((ms & 1) * TS_HAND + 0) * TS;   // hand-over buffer of this slab, distance 1
-    if (kp >= 1) {
-      if (fed_by_prev_local) {
-        if (tid < TS) {                            // the peer stores the 64 unknowns straight into xc
-          unsigned spins = 0;
-          while (unpublished(ld_shared_relaxed_f64(xc + tid))) {
-            if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
-          }
+    if constexpr (R == 1) {
+      if (owner) {
+        double a;
+        if (FWD) {
+          a = acc[ms * TS + idx];
+        } else {                                     // the eight warps' partial sums, in a fixed order
+          const double* p = acc + ms * 8 * TS + idx;
+          a = ((p[0] + p[TS]) + (p[2 * TS] + p[3 * TS])) + ((p[4 * TS] + p[5 * TS]) + (p[6 * TS] + p[7 * TS]));
         }
-      } else {
-        const double* src = P.xpub + (int64_t)(kp - 1) * TS;
-        if (tid < TS) {
-          double v = ld_relaxed_f64(src + tid);
-          unsigned spins = 0;
-          while (unpublished(v)) {
-            if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
-            v = ld_relaxed_f64(src + tid);
-          }
-          xc[tid] = v;
-        }
+        vs[idx] = (idx < w) ? bs[idx] - a : 0.0;
       }
+      mbar_wait(&full[0], dphase);
+      dphase ^= 1;
       __syncthreads();
-      TRSV_STAMP(kp, 0);
-      xv -= matvec(wtile, xc, FWD ? TS : blkw(kp - 1));
-    }
-    if (owner) {
-      if (unpublished(xv)) xv = __longlong_as_double(0x7ff8000000000000ll);   // never publish the sentinel
-#pragma unroll
-      for (int d = 1; d <= TS_HAND; ++d) {         // first the hops that are on (or next to) the serial chain
-        if (local_to(d) && kp + d < nb) {
-          // the peer's slab kp + d is its slab number (kp + d) / G: that parity selects its buffer set
-          double* dst = xh + ((((kp + d) / G) & 1) * TS_HAND + (d - 1)) * TS + idx;
-          st_remote_f64(map_to_cta(smem_addr(dst), (uint32_t)(peer_ahead(d) % CS)), xv);
+      double xv = matvec(dtile, vs, TS);
+      double* xc = xh + ((ms & 1) * TS_HAND + 0) * TS;   // hand-over buffer of this slab, distance 1
+      if (kp >= 1) {
+        if (fed_by_prev_local) {
+          if (tid < TS) {                            // the peer stores the 64 unknowns straight into xc
+            unsigned spins = 0;
+            while (unpublished(ld_shared_relaxed_f64(xc + tid))) {
+              if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
+            }
+          }
+        } else {
+          const double* src = P.xpub + (int64_t)(kp - 1) * TS;
+          if (tid < TS) {
+            double v = ld_relaxed_f64(src + tid);
+            unsigned spins = 0;
+            while (unpublished(v)) {
+              if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
+              v = ld_relaxed_f64(src + tid);
+            }
+            xc[tid] = v;
+          }
+        }
+        __syncthreads();
+        TRSV_STAMP(kp, 0);
+        xv -= matvec(wtile, xc, FWD ? TS : blkw(kp - 1));
+      }
+      if (owner) {
+        if (unpublished(xv)) xv = __longlong_as_double(0x7ff8000000000000ll);   // never publish the sentinel
+  #pragma unroll
+        for (int d = 1; d <= TS_HAND; ++d) {         // first the hops that are on (or next to) the serial chain
+          if (local_to(d) && kp + d < nb) {
+            // the peer's slab kp + d is its slab number (kp + d) / G: that parity selects its buffer set
+            double* dst = xh + ((((kp + d) / G) & 1) * TS_HAND + (d - 1)) * TS + idx;
+            st_remote_f64(map_to_cta(smem_addr(dst), (uint32_t)(peer_ahead(d) % CS)), xv);
+          }
+        }
+        st_relaxed_f64(P.xpub + (int64_t)kp * TS + idx, xv);
+        if (idx < w) P.b[r0 + idx] = xv;
+      }
+    } else {
+      if (owner) {
+  #pragma unroll
+        for (int c = 0; c < R; ++c) {
+          double a;
+          if (FWD) {
+            a = acc[(ms * R + c) * TS + idx];
+          } else {                                   // the eight warps' partial sums, in a fixed order
+            const double* p = acc + (ms * 8 * R + c) * TS + idx;
+            constexpr int W = R * TS;                // from one warp's partials to the next
+            a = ((p[0] + p[W]) + (p[2 * W] + p[3 * W])) + ((p[4 * W] + p[5 * W]) + (p[6 * W] + p[7 * W]));
+          }
+          vs[c * TS + idx] = (idx < w) ? bs[c * TS + idx] - a : 0.0;
         }
       }
-      st_relaxed_f64(P.xpub + (int64_t)kp * TS + idx, xv);
-      if (idx < w) P.b[r0 + idx] = xv;
+      mbar_wait(&full[0], dphase);
+      dphase ^= 1;
+      __syncthreads();
+      double xv[R];
+  #pragma unroll
+      for (int c = 0; c < R; ++c) xv[c] = matvec(dtile, vs + c * TS, TS);
+      double* xc = xh + ((ms & 1) * TS_HAND + 0) * TS * R;   // hand-over buffer of this slab, distance 1
+      if (kp >= 1) {
+        if (fed_by_prev_local) {
+          if (tid < TS) {                            // the peer stores the 64 unknowns straight into xc
+  #pragma unroll
+            for (int c = 0; c < R; ++c) {
+              unsigned spins = 0;
+              while (unpublished(ld_shared_relaxed_f64(xc + c * TS + tid))) {
+                if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
+              }
+            }
+          }
+        } else {
+          const double* src = P.xpub + (int64_t)(kp - 1) * TS * R;
+          if (tid < TS) {
+  #pragma unroll
+            for (int c = 0; c < R; ++c) {
+              double v = ld_relaxed_f64(src + c * TS + tid);
+              unsigned spins = 0;
+              while (unpublished(v)) {
+                if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
+                v = ld_relaxed_f64(src + c * TS + tid);
+              }
+              xc[c * TS + tid] = v;
+            }
+          }
+        }
+        __syncthreads();
+        TRSV_STAMP(kp, 0);
+  #pragma unroll
+        for (int c = 0; c < R; ++c) xv[c] -= matvec(wtile, xc + c * TS, FWD ? TS : blkw(kp - 1));
+      }
+      if (owner) {
+  #pragma unroll
+        for (int c = 0; c < R; ++c) {
+          if (unpublished(xv[c])) xv[c] = __longlong_as_double(0x7ff8000000000000ll);   // never publish the sentinel
+  #pragma unroll
+          for (int d = 1; d <= TS_HAND; ++d) {       // first the hops that are on (or next to) the serial chain
+            if (local_to(d) && kp + d < nb) {
+              // the peer's slab kp + d is its slab number (kp + d) / G: that parity selects its buffer set
+              double* dst = xh + ((((kp + d) / G) & 1) * TS_HAND + (d - 1)) * TS * R + c * TS + idx;
+              st_remote_f64(map_to_cta(smem_addr(dst), (uint32_t)(peer_ahead(d) % CS)), xv[c]);
+            }
+          }
+          st_relaxed_f64(P.xpub + (int64_t)kp * TS * R + c * TS + idx, xv[c]);
+          if (idx < w) P.b[c * P.ld + r0 + idx] = xv[c];
+        }
+      }
     }
     TRSV_STAMP(kp, 2);
     __syncthreads();                               // dtile, wtile, bs, vs, xc are free again
     // re-arm this slab's hand-over buffer: the next store into it (slab ms + 2) causally follows the publication of
     // slab ms + 1 by this CTA, which follows this line in program order
     if (CS > 1) {
-      double* mine = xh + (ms & 1) * TS_HAND * TS;
-      for (int i = tid; i < TS_HAND * TS; i += TS_THREADS) mine[i] = __longlong_as_double(-1ll);
+      double* mine = xh + (ms & 1) * TS_HAND * TS * R;
+      for (int i = tid; i < TS_HAND * TS * R; i += TS_THREADS) mine[i] = __longlong_as_double(-1ll);
     }
     prefetch_solve(ms + 1);
   };
@@ -436,55 +516,118 @@ trsv_sweep_kernel(TrsvParams P) {
 #pragma unroll
       for (int g = 0; g < TS_WIN; ++g)
         v[i][g] = (g < cnt && r0 + i < N) ? ldg2(base + (int64_t)i * ld + g * TS, vec) : make_double2(0.0, 0.0);
-    double s[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      double a0 = 0.0, a1 = 0.0;
-#pragma unroll
-      for (int g = 0; g < TS_WIN; ++g) {
-        if (g < cnt) {
-          a0 = fma(v[i][g].x, xs[g * TS + 2 * lane], a0);
-          a1 = fma(v[i][g].y, xs[g * TS + 2 * lane + 1], a1);
+    if constexpr (R == 1) {
+      double s[8];
+  #pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        double a0 = 0.0, a1 = 0.0;
+  #pragma unroll
+        for (int g = 0; g < TS_WIN; ++g) {
+          if (g < cnt) {
+            a0 = fma(v[i][g].x, xs[g * TS + 2 * lane], a0);
+            a1 = fma(v[i][g].y, xs[g * TS + 2 * lane + 1], a1);
+          }
+        }
+        s[i] = a0 + a1;
+      }
+  #pragma unroll
+      for (int o = 16; o > 0; o >>= 1)
+  #pragma unroll
+        for (int i = 0; i < 8; ++i) s[i] += __shfl_xor_sync(0xffffffffu, s[i], o);
+      if (lane < 8) {
+        double sv = s[0];
+  #pragma unroll
+        for (int i = 1; i < 8; ++i) sv = (lane == i) ? s[i] : sv;
+        acc[m * TS + warp * 8 + lane] += sv;
+      }
+    } else {
+  #pragma unroll
+      for (int c = 0; c < R; ++c) {                  // the rows are read once; the columns are accumulated one by one
+        double s[8];
+  #pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          double a0 = 0.0, a1 = 0.0;
+  #pragma unroll
+          for (int g = 0; g < TS_WIN; ++g) {
+            if (g < cnt) {
+              a0 = fma(v[i][g].x, xs[(g * R + c) * TS + 2 * lane], a0);
+              a1 = fma(v[i][g].y, xs[(g * R + c) * TS + 2 * lane + 1], a1);
+            }
+          }
+          s[i] = a0 + a1;
+        }
+  #pragma unroll
+        for (int o = 16; o > 0; o >>= 1)
+  #pragma unroll
+          for (int i = 0; i < 8; ++i) s[i] += __shfl_xor_sync(0xffffffffu, s[i], o);
+        if (lane < 8) {
+          double sv = s[0];
+  #pragma unroll
+          for (int i = 1; i < 8; ++i) sv = (lane == i) ? s[i] : sv;
+          acc[(m * R + c) * TS + warp * 8 + lane] += sv;
         }
       }
-      s[i] = a0 + a1;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1)
-#pragma unroll
-      for (int i = 0; i < 8; ++i) s[i] += __shfl_xor_sync(0xffffffffu, s[i], o);
-    if (lane < 8) {
-      double sv = s[0];
-#pragma unroll
-      for (int i = 1; i < 8; ++i) sv = (lane == i) ? s[i] : sv;
-      acc[m * TS + warp * 8 + lane] += sv;
     }
   };
   auto visit_bwd = [&](int m, int j0, int cnt) {
     const int kp = c + m * G;
     const int64_t c0 = blk0(kp) + 2 * lane;          // the slab's columns
-    double a0 = 0.0, a1 = 0.0, b0 = 0.0, b1 = 0.0;
-    for (int g = 0; g < cnt; ++g) {
-      const int64_t rb = blk0(j0 + g);               // rows of window block g (primed j0 + g)
-      const int rows = blkw(j0 + g);
-      double2 v[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const int r = warp * 8 + i;
-        v[i] = (r < rows) ? ldg2(P.L + (rb + r) * ld + c0, vec) : make_double2(0.0, 0.0);
+    if constexpr (R == 1) {
+      double a0 = 0.0, a1 = 0.0, b0 = 0.0, b1 = 0.0;
+      for (int g = 0; g < cnt; ++g) {
+        const int64_t rb = blk0(j0 + g);               // rows of window block g (primed j0 + g)
+        const int rows = blkw(j0 + g);
+        double2 v[8];
+  #pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const int r = warp * 8 + i;
+          v[i] = (r < rows) ? ldg2(P.L + (rb + r) * ld + c0, vec) : make_double2(0.0, 0.0);
+        }
+  #pragma unroll
+        for (int i = 0; i < 8; i += 2) {
+          const double x0 = xs[g * TS + warp * 8 + i], x1 = xs[g * TS + warp * 8 + i + 1];
+          a0 = fma(v[i].x, x0, a0);
+          a1 = fma(v[i].y, x0, a1);
+          b0 = fma(v[i + 1].x, x1, b0);
+          b1 = fma(v[i + 1].y, x1, b1);
+        }
       }
-#pragma unroll
-      for (int i = 0; i < 8; i += 2) {
-        const double x0 = xs[g * TS + warp * 8 + i], x1 = xs[g * TS + warp * 8 + i + 1];
-        a0 = fma(v[i].x, x0, a0);
-        a1 = fma(v[i].y, x0, a1);
-        b0 = fma(v[i + 1].x, x1, b0);
-        b1 = fma(v[i + 1].y, x1, b1);
+      double* p = acc + (m * 8 + warp) * TS + 2 * lane;
+      p[0] += a0 + b0;
+      p[1] += a1 + b1;
+    } else {
+      double a0[R], a1[R], b0[R], b1[R];
+  #pragma unroll
+      for (int c = 0; c < R; ++c) a0[c] = a1[c] = b0[c] = b1[c] = 0.0;
+      for (int g = 0; g < cnt; ++g) {
+        const int64_t rb = blk0(j0 + g);               // rows of window block g (primed j0 + g)
+        const int rows = blkw(j0 + g);
+        double2 v[8];
+  #pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const int r = warp * 8 + i;
+          v[i] = (r < rows) ? ldg2(P.L + (rb + r) * ld + c0, vec) : make_double2(0.0, 0.0);
+        }
+  #pragma unroll
+        for (int c = 0; c < R; ++c) {
+          const double* xg = xs + (g * R + c) * TS + warp * 8;
+  #pragma unroll
+          for (int i = 0; i < 8; i += 2) {
+            const double x0 = xg[i], x1 = xg[i + 1];
+            a0[c] = fma(v[i].x, x0, a0[c]);
+            a1[c] = fma(v[i].y, x0, a1[c]);
+            b0[c] = fma(v[i + 1].x, x1, b0[c]);
+            b1[c] = fma(v[i + 1].y, x1, b1[c]);
+          }
+        }
+      }
+  #pragma unroll
+      for (int c = 0; c < R; ++c) {
+        double* p = acc + ((m * 8 + warp) * R + c) * TS + 2 * lane;
+        p[0] += a0[c] + b0[c];
+        p[1] += a1[c] + b1[c];
       }
     }
-    double* p = acc + (m * 8 + warp) * TS + 2 * lane;
-    p[0] += a0 + b0;
-    p[1] += a1 + b1;
   };
 
   // L2 prefetch of the 64-row tiles of slab index ms against column blocks j0 .. j0 + cnt - 1: near the chain front
@@ -511,42 +654,80 @@ trsv_sweep_kernel(TrsvParams P) {
   // fetch the unknowns of column blocks j0 .. j0 + cnt - 1 into xs (urgent: all 64 threads poll from the start)
   auto fetch_window = [&](int j0, int cnt, bool urgent) {
     __syncthreads();                               // everyone is done with the previous window
-    const double* src = P.xpub + (int64_t)j0 * TS;
-    if (!urgent) {
-      if (tid == 0) {                              // blocks are published in order: wait for the last one, lazily
-        unsigned spins = 0;
-        while (unpublished(ld_relaxed_f64(src + (cnt - 1) * TS))) {
-          if (spins > 16u) __nanosleep(32);
-          if (++spins > (1u << 23)) { atomicExch(&g_tgp_device_error, 1); break; }
+    if constexpr (R == 1) {
+      const double* src = P.xpub + (int64_t)j0 * TS;
+      if (!urgent) {
+        if (tid == 0) {                              // blocks are published in order: wait for the last one, lazily
+          unsigned spins = 0;
+          while (unpublished(ld_relaxed_f64(src + (cnt - 1) * TS))) {
+            if (spins > 16u) __nanosleep(32);
+            if (++spins > (1u << 23)) { atomicExch(&g_tgp_device_error, 1); break; }
+          }
         }
+        __syncthreads();
+      }
+      if (tid < cnt * TS) {
+        double v = ld_relaxed_f64(src + tid);
+        unsigned spins = 0;
+        while (unpublished(v)) {
+          if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
+          v = ld_relaxed_f64(src + tid);
+        }
+        if (!FWD && (tid & 63) >= blkw(j0 + (tid >> 6))) v = 0.0;    // padding rows of a short block
+        xs[tid] = v;
+      }
+      __syncthreads();
+    } else {
+      const double* src = P.xpub + (int64_t)j0 * TS * R;
+      if (!urgent) {
+        if (tid == 0) {                              // blocks are published in order: wait for the last one, lazily
+          unsigned spins = 0;
+          while (unpublished(ld_relaxed_f64(src + (cnt - 1) * TS * R))) {
+            if (spins > 16u) __nanosleep(32);
+            if (++spins > (1u << 23)) { atomicExch(&g_tgp_device_error, 1); break; }
+          }
+        }
+        __syncthreads();
+      }
+      for (int i = tid; i < cnt * TS * R; i += TS_THREADS) {
+        double v = ld_relaxed_f64(src + i);
+        unsigned spins = 0;
+        while (unpublished(v)) {
+          if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
+          v = ld_relaxed_f64(src + i);
+        }
+        if (!FWD && (i & 63) >= blkw(j0 + i / (TS * R))) v = 0.0;    // padding rows of a short block
+        xs[i] = v;
       }
       __syncthreads();
     }
-    if (tid < cnt * TS) {
-      double v = ld_relaxed_f64(src + tid);
-      unsigned spins = 0;
-      while (unpublished(v)) {
-        if (++spins > (1u << 25)) { atomicExch(&g_tgp_device_error, 1); break; }
-        v = ld_relaxed_f64(src + tid);
-      }
-      if (!FWD && (tid & 63) >= blkw(j0 + (tid >> 6))) v = 0.0;    // padding rows of a short block
-      xs[tid] = v;
-    }
-    __syncthreads();
   };
 
   // the unknowns of the block at distance d before slab index ms's diagonal, handed over by a cluster peer
   auto fetch_handover = [&](int ms, int d) {
     __syncthreads();                               // everyone is done with the previous window
-    const double* src = xh + ((ms & 1) * TS_HAND + (d - 1)) * TS;
-    if (tid < TS) {
-      unsigned spins = 0;
-      double v = ld_shared_relaxed_f64(src + tid);
-      while (unpublished(v)) {
-        if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
-        v = ld_shared_relaxed_f64(src + tid);
+    if constexpr (R == 1) {
+      const double* src = xh + ((ms & 1) * TS_HAND + (d - 1)) * TS;
+      if (tid < TS) {
+        unsigned spins = 0;
+        double v = ld_shared_relaxed_f64(src + tid);
+        while (unpublished(v)) {
+          if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
+          v = ld_shared_relaxed_f64(src + tid);
+        }
+        xs[tid] = v;                                 // (a short block's padding rows are published as zeros)
       }
-      xs[tid] = v;                                 // (a short block's padding rows are published as zeros)
+    } else {
+      const double* src = xh + ((ms & 1) * TS_HAND + (d - 1)) * TS * R;
+      for (int i = tid; i < TS * R; i += TS_THREADS) {
+        unsigned spins = 0;
+        double v = ld_shared_relaxed_f64(src + i);
+        while (unpublished(v)) {
+          if (++spins > (1u << 26)) { atomicExch(&g_tgp_device_error, 2); break; }
+          v = ld_shared_relaxed_f64(src + i);
+        }
+        xs[i] = v;                                   // (a short block's padding rows are published as zeros)
+      }
     }
     __syncthreads();
   };
@@ -594,9 +775,9 @@ trsv_sweep_kernel(TrsvParams P) {
   if (CS > 1) cluster_sync_all();                  // shared memory of a CTA stays valid while peers may still write
 }
 
-static size_t trsv_smem_bytes(bool fwd, int slabs_per_cta) {
-  return (size_t)2 * TS_TILE_D * 8 + (size_t)(TS_WIN * TS + 2 * TS_HAND * TS + 2 * TS + 4 * TS) * 8 + 2 * 8 +
-         (size_t)slabs_per_cta * TS * 8 * (fwd ? 1 : 8);
+static size_t trsv_smem_bytes(bool fwd, int slabs_per_cta, int R = 1) {
+  return (size_t)2 * TS_TILE_D * 8 + (size_t)((TS_WIN * TS + 2 * TS_HAND * TS + 2 * TS) * R + 4 * TS) * 8 + 2 * 8 +
+         (size_t)slabs_per_cta * TS * 8 * (fwd ? 1 : 8) * R;
 }
 
 static int g_trsv_cluster = -1;   // option "trsv_cluster": -1 automatic, 1 no clusters, 2 / 4 / 8 cluster size
@@ -604,7 +785,7 @@ extern "C" int tgp_trsv_set_cluster(int v) { g_trsv_cluster = v; return TGP_OK; 
 
 // CTAs of one cooperative launch: as many as are co-resident (one per SM: the kernel takes most of the shared
 // memory), in clusters of CS when a cluster size is in use.
-template <bool FWD>
+template <bool FWD, int R>
 static int trsv_grid(int nb, int cs, size_t smem) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)cs);
@@ -618,7 +799,7 @@ static int trsv_grid(int nb, int cs, size_t smem) {
   cfg.attrs = at;
   cfg.numAttrs = 1;
   int nclusters = 0;
-  if (cudaOccupancyMaxActiveClusters(&nclusters, trsv_sweep_kernel<FWD>, &cfg) != cudaSuccess) {
+  if (cudaOccupancyMaxActiveClusters(&nclusters, trsv_sweep_kernel<FWD, R>, &cfg) != cudaSuccess) {
     cudaGetLastError();
     return 0;
   }
@@ -627,14 +808,20 @@ static int trsv_grid(int nb, int cs, size_t smem) {
   return g < want ? g : want;
 }
 
-template <bool FWD>
-static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
-  TrsvParams P = P0;
+template <bool FWD, int R>
+static void trsv_max_smem() {
   static TgpPerDeviceOnce once;
   if (tgp_first_use_on_device(once))
-    TGP_CUDA(cudaFuncSetAttribute(trsv_sweep_kernel<FWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    cudaFuncSetAttribute(trsv_sweep_kernel<FWD, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+}
+
+// Grid of the single right-hand-side sweep: cluster size CS and CTA count G.
+template <bool FWD>
+static void trsv_config(const TrsvParams& P, int& cs, int& G) {
+  trsv_max_smem<FWD, 1>();
   // cluster size: the largest of 8 / 4 / 2 that still keeps (nearly) all SMs busy; none for tiny matrices
-  int cs = 1, G = P.G;
+  cs = 1;
+  G = P.G;
   const size_t smem1 = trsv_smem_bytes(FWD, (P.nb + P.G - 1) / P.G);
   if (g_trsv_cluster != 1 && P.nb >= 4) {
     const int tries[3] = {8, 4, 2};
@@ -642,7 +829,7 @@ static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
       const int c2 = tries[t];
       if (g_trsv_cluster > 1 && c2 != g_trsv_cluster) continue;
       if (P.nb < c2) continue;
-      const int g = trsv_grid<FWD>(P.nb, c2, smem1 + 4096);
+      const int g = trsv_grid<FWD, 1>(P.nb, c2, smem1 + 4096);
       if (g >= c2 && (g_trsv_cluster > 1 || 10 * g >= 9 * (P.nb < P.G ? (P.nb / c2) * c2 : P.G))) {
         cs = c2;
         G = g;
@@ -650,9 +837,19 @@ static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
       }
     }
   }
+}
+
+// R > 1 runs on exactly the grid of R = 1 (the caller checks trsv_fits first): the slabs, their windows and hence every
+// column's order of accumulation are those of the single right-hand-side sweep.
+template <bool FWD, int R>
+static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
+  TrsvParams P = P0;
+  int cs, G;
+  trsv_config<FWD>(P, cs, G);
   P.CS = cs;
   P.G = G;
-  const size_t smem = trsv_smem_bytes(FWD, (P.nb + P.G - 1) / P.G);
+  const size_t smem = trsv_smem_bytes(FWD, (P.nb + P.G - 1) / P.G, R);
+  if (R > 1) trsv_max_smem<FWD, R>();
   TGP_CHECK_ARG(smem <= 227 * 1024, "matrix too large for the sweep kernel's per-CTA accumulators");
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)P.G);
@@ -668,11 +865,11 @@ static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
   at[1].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = cs > 1 ? 2 : 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, trsv_sweep_kernel<FWD>, P);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, trsv_sweep_kernel<FWD, R>, P);
   if (e != cudaSuccess && cs > 1) {                // clusters + cooperative launch refused: go on without clusters
     cudaGetLastError();
     g_trsv_cluster = 1;
-    return trsv_launch<FWD>(P0, st);
+    return trsv_launch<FWD, R>(P0, st);
   }
   TGP_CUDA(e);
   return TGP_OK;
@@ -698,10 +895,45 @@ static cudaMemPool_t trsv_pool() {
   return pools[dev];
 }
 
+// Can R columns run on the grid of the single-column sweep (shared memory, co-residency)?
+template <bool FWD, int R>
+static bool trsv_fits(const TrsvParams& P) {
+  int cs, G;
+  trsv_config<FWD>(P, cs, G);
+  const size_t smem = trsv_smem_bytes(FWD, (P.nb + G - 1) / G, R);
+  if (smem > 227 * 1024) return false;
+  trsv_max_smem<FWD, R>();
+  return trsv_grid<FWD, R>(P.nb, cs, smem) >= G;
+}
+
+template <bool FWD>
+static bool trsv_fits_r(const TrsvParams& P, int R) {
+  switch (R) {
+    case 2: return trsv_fits<FWD, 2>(P);
+    case 4: return trsv_fits<FWD, 4>(P);
+    case 8: return trsv_fits<FWD, 8>(P);
+    default: return true;
+  }
+}
+
+template <bool FWD>
+static int trsv_launch_r(const TrsvParams& P, int R, cudaStream_t st) {
+  switch (R) {
+    case 1: return trsv_launch<FWD, 1>(P, st);
+    case 2: return trsv_launch<FWD, 2>(P, st);
+    case 4: return trsv_launch<FWD, 4>(P, st);
+    default: return trsv_launch<FWD, 8>(P, st);
+  }
+}
+
 // Workspace layout: [nb * 4096 doubles: inverse diagonal blocks][nb * 4096: W (forward)][nb * 4096: M (backward)]
-// [2 * nb * 64 doubles: published unknowns of the forward and of the backward sweep, filled with 0xFF bytes =
-// "not yet published"].  which = 1: forward only, 2: backward only, 3: both (forward then backward).
-int tgp_trsv_sweeps(const double* L, int64_t N, int64_t ld, double* b, int which, cudaStream_t st) {
+// [2 * nb * 64 * Rmax doubles: published unknowns of the forward and of the backward sweep, filled with 0xFF bytes =
+// "not yet published"][Rmax * ld: the right-hand sides of a multi-column sweep, padded with zero columns].
+// which = 1: forward only, 2: backward only, 3: both (forward then backward).
+// r columns b + c ld (c < r <= TGP_MAX_RHS) are swept in groups of R = 8, 4 or 2 columns (the largest that holds them
+// and fits the single-column grid, else fewer), one column at a time when r == 1.  The diagonal-block inverses are
+// computed once for all of them.
+static int trsv_sweeps_impl(const double* L, int64_t N, int64_t ld, double* b, int r, int which, cudaStream_t st) {
   if (N <= 0) return TGP_OK;
   const int nb = (int)tgp_cdiv(N, TS);
   const int sms = tgp_num_sms();
@@ -710,27 +942,25 @@ int tgp_trsv_sweeps(const double* L, int64_t N, int64_t ld, double* b, int which
   P.G = nb < sms ? nb : sms;
   P.CS = 1;
   P.aligned = ((ld & 1) == 0) && ((((uintptr_t)L) & 15) == 0);
+  int rmax = 1;
+  while (rmax < r) rmax *= 2;
   const size_t blk_d = (size_t)nb * TS * TS;
-  const size_t pub_d = (size_t)2 * nb * TS;
+  const size_t pub_d = (size_t)2 * nb * TS * rmax;
+  const size_t rhs_d = rmax > 1 ? (size_t)rmax * ld : 0;
   cudaMemPool_t pool = trsv_pool();
   if (!pool) {
     tgp_set_error("tgp_trsv_sweeps: cudaMemPoolCreate failed: %s", cudaGetErrorString(cudaGetLastError()));
     return TGP_ERR_CUDA;
   }
   void* ws = nullptr;
-  TGP_CUDA(cudaMallocFromPoolAsync(&ws, (3 * blk_d + pub_d) * sizeof(double), pool, st));
+  TGP_CUDA(cudaMallocFromPoolAsync(&ws, (3 * blk_d + pub_d + rhs_d) * sizeof(double), pool, st));
   double* dinv = reinterpret_cast<double*>(ws);
   double* wf = dinv + blk_d;
   double* wb = wf + blk_d;
   double* xpub = wb + blk_d;
+  double* rhs = xpub + pub_d;
   int rc = TGP_OK;
   do {
-#ifdef TGP_TRSV_TIMING
-    // which & 4 (debug): pretend every block is already published -> no dependency waits, pure streaming rate
-    if (cudaMemsetAsync(xpub, (which & 4) ? 0 : 0xFF, pub_d * sizeof(double), st) != cudaSuccess) { rc = TGP_ERR_CUDA; break; }
-#else
-    if (cudaMemsetAsync(xpub, 0xFF, pub_d * sizeof(double), st) != cudaSuccess) { rc = TGP_ERR_CUDA; break; }
-#endif
     static TgpPerDeviceOnce prep_once;
     if (tgp_first_use_on_device(prep_once) &&
         cudaFuncSetAttribute(trsv_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TP_SMEM) != cudaSuccess) {
@@ -741,22 +971,61 @@ int tgp_trsv_sweeps(const double* L, int64_t N, int64_t ld, double* b, int which
                                                          (which & 2) ? wb : nullptr);
     if (cudaGetLastError() != cudaSuccess) { rc = TGP_ERR_CUDA; break; }
     P.dinv = dinv;
-    if (which & 1) {
-      P.wmat = wf;
-      P.xpub = xpub;
-      rc = trsv_launch<true>(P, st);
-      if (rc) break;
-    }
-    if (which & 2) {
-      P.wmat = wb;
-      P.xpub = xpub + (size_t)nb * TS;
-      rc = trsv_launch<false>(P, st);
-      if (rc) break;
+    // the widest group of columns whose sweeps run on the single-column grid
+    int rfit = rmax;
+    while (rfit > 1 && !(((which & 1) == 0 || trsv_fits_r<true>(P, rfit)) &&
+                         ((which & 2) == 0 || trsv_fits_r<false>(P, rfit))))
+      rfit /= 2;
+    for (int c0 = 0, R = 1; c0 < r; c0 += R) {
+      R = 1;
+      while (R < r - c0 && R < rfit) R *= 2;
+      const int nc = (r - c0 < R) ? r - c0 : R;
+      if (R > 1) {                                 // the group's columns, padded with zero columns, at pitch ld
+        if (cudaMemsetAsync(rhs, 0, (size_t)R * ld * sizeof(double), st) != cudaSuccess ||
+            cudaMemcpy2DAsync(rhs, ld * sizeof(double), b + (size_t)c0 * ld, ld * sizeof(double), N * sizeof(double),
+                              nc, cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+          rc = TGP_ERR_CUDA;
+          break;
+        }
+      }
+      P.b = R > 1 ? rhs : b + (size_t)c0 * ld;
+#ifdef TGP_TRSV_TIMING
+      // which & 4 (debug): pretend every block is already published -> no dependency waits, pure streaming rate
+      if (cudaMemsetAsync(xpub, (which & 4) ? 0 : 0xFF, pub_d * sizeof(double), st) != cudaSuccess) { rc = TGP_ERR_CUDA; break; }
+#else
+      if (cudaMemsetAsync(xpub, 0xFF, pub_d * sizeof(double), st) != cudaSuccess) { rc = TGP_ERR_CUDA; break; }
+#endif
+      if (which & 1) {
+        P.wmat = wf;
+        P.xpub = xpub;
+        rc = trsv_launch_r<true>(P, R, st);
+        if (rc) break;
+      }
+      if (which & 2) {
+        P.wmat = wb;
+        P.xpub = xpub + (size_t)nb * TS * R;
+        rc = trsv_launch_r<false>(P, R, st);
+        if (rc) break;
+      }
+      if (R > 1 && cudaMemcpy2DAsync(b + (size_t)c0 * ld, ld * sizeof(double), rhs, ld * sizeof(double),
+                                     N * sizeof(double), nc, cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        rc = TGP_ERR_CUDA;
+        break;
+      }
     }
   } while (0);
   if (rc == TGP_ERR_CUDA) tgp_set_error("tgp_trsv_sweeps: %s", cudaGetErrorString(cudaGetLastError()));
   cudaFreeAsync(ws, st);
   return rc;
+}
+
+int tgp_trsv_sweeps(const double* L, int64_t N, int64_t ld, double* b, int which, cudaStream_t st) {
+  return trsv_sweeps_impl(L, N, ld, b, 1, which, st);
+}
+
+// r right-hand sides b + c ld, c < r (1 <= r <= TGP_MAX_RHS): one pass over the factor per group of columns.
+int tgp_trsv_sweeps_multi(const double* L, int64_t N, int64_t ld, double* b, int r, int which, cudaStream_t st) {
+  return trsv_sweeps_impl(L, N, ld, b, r, which, st);
 }
 
 #ifdef TGP_TRSV_TIMING

@@ -25,6 +25,11 @@ from .two_pcf import two_pcf
 class GPInterpolation(object):
     """Gaussian-process interpolation of one scalar surface sampled at scattered 1-D or 2-D positions.
 
+    Several outputs (extension): a y of shape (n, r), 1 <= r <= 8, holds r fields measured at the same points with
+    the same errors.  They are interpolated as r independent GPs sharing one kernel (scikit-learn's
+    GaussianProcessRegressor with multi-target y): one factorisation serves all of them, predictions are (m, r), the
+    log-likelihood is the sum over the outputs and "log-likelihood" fits the shared kernel to all of them together.
+
     Constructor keywords (names, order and defaults as in the reference):
 
     kernel          kernel string, evaluated by `eval_kernel` (e.g. "4.0 * AnisotropicRBF(invLam=array(...))")
@@ -83,6 +88,7 @@ class GPInterpolation(object):
             X0, y0 = None, None
         self._X0 = X0
         self._y0 = y0
+        self._has_average = average_fits is not None
         self._alpha = None
         self._factor = None
 
@@ -142,7 +148,7 @@ class GPInterpolation(object):
         self._ensure_solved(self._y - self._mean - self._spatial_average, self._X, self.kernel, self._y_err)
         Xd, desc, ws = self._factor
         Xs = backend.as_points(X)
-        mean = backend.predict_mean(Xs, Xd, desc, self._alpha_dev)
+        mean = self._predict_mean(Xs, Xd, desc)
         var, self._var_plan = None, {}
         if self.WINDOWED_VARIANCE:
             var = backend.predict_var_windowed(Xs, Xd, desc, self._e2_dev, chunk=self.VAR_CHUNK, stats=self._var_plan)
@@ -152,15 +158,22 @@ class GPInterpolation(object):
         y = mean.cpu().numpy() + self._mean + self._build_average_meanify(X)
         return y, var.cpu().numpy()
 
+    def _predict_mean(self, Xs, Xd, desc):
+        """K(Xs, X) alpha on the device: (m,), or (m, r) for several outputs."""
+        if self._alpha_dev.dim() == 2:
+            return backend.predict_mean_multi(Xs, Xd, desc, self._alpha_dev)
+        return backend.predict_mean(Xs, Xd, desc, self._alpha_dev)
+
     def _ensure_solved(self, y, X1, kernel, y_err):
-        """K + diag(y_err^2) -> L -> alpha on the device, cached like ``_alpha`` (gp_interp.py:179-182)."""
+        """K + diag(y_err^2) -> L -> alpha on the device, cached like ``_alpha`` (gp_interp.py:179-182).  A y of
+        shape (n, r) gives alpha (n, r) from the same factorisation (tgp_loglike_multi)."""
         if self._alpha is not None and self._factor is not None:
             return
         Xd = backend.as_points(X1)
         n = Xd.shape[0]
         desc = lower(kernel, Xd.shape[1])
         e2 = backend.to_device(np.asarray(y_err, dtype=np.float64).reshape(-1) ** 2)
-        yd = backend.to_device(np.asarray(y, dtype=np.float64).reshape(-1))
+        yd = _device_outputs(y)
         # A kernel whose support is short against the field: with the points sorted along one axis K is zero (below
         # 1e-40 amp) outside an envelope that its Cholesky factor keeps -- factorise inside it (N bw^2 flop instead of
         # N^3 / 3).  The factor, X and alpha are then held in the sorted order; `_alpha` (host) in the caller's.
@@ -169,8 +182,8 @@ class GPInterpolation(object):
             Xd, yd, e2 = Xd[env["order"]].contiguous(), yd[env["order"]].contiguous(), e2[env["order"]].contiguous()
         # one call: K (lower) -> L with y riding through the factorisation as an extra row (forward substitution
         # for free), then the backward sweep (tgp_loglike, want_alpha)
-        _, info, alpha, ws = backend.loglike(Xd, yd, e2, desc, want_alpha=True,
-                                             row_end=None if env is None else env["row_end"])
+        loglike = backend.loglike_multi if yd.dim() == 2 else backend.loglike
+        _, info, alpha, ws = loglike(Xd, yd, e2, desc, want_alpha=True, row_end=None if env is None else env["row_end"])
         bad = int(info.item())
         if bad < 0:
             raise _cabi.TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % bad)
@@ -194,8 +207,12 @@ class GPInterpolation(object):
         Z = (K + diag(y_err^2))^-1 (its diagonal from the selected inverse, tgp_selinv), y_err after the white noise.
         This is what predict / predict_var return at X_i from the other N - 1 points with the same kernel; the
         normalising mean and the mean function keep their all-point values and are added back as predict does.
-        Factorises into a workspace of its own: the cached factor of predict_var / return_cov stays as it is."""
-        y = np.asarray(self._y - self._mean - self._spatial_average, dtype=np.float64).reshape(-1)
+        Factorises into a workspace of its own: the cached factor of predict_var / return_cov stays as it is.
+        Several outputs: mean (n, r) with mean_ic = y_ic - alpha_ic / Z_ii, var (n,) shared by the outputs."""
+        y = np.asarray(self._y - self._mean - self._spatial_average, dtype=np.float64)
+        multi = y.ndim == 2
+        if not multi:
+            y = y.reshape(-1)
         Xd = backend.as_points(self._X)
         n = Xd.shape[0]
         desc = lower(self.kernel, Xd.shape[1])
@@ -205,7 +222,8 @@ class GPInterpolation(object):
         if env is not None:
             Xd, yd, e2 = Xd[env["order"]].contiguous(), yd[env["order"]].contiguous(), e2[env["order"]].contiguous()
         row_end = None if env is None else env["row_end"]
-        _, info, alpha, ws = backend.loglike(Xd, yd, e2, desc, want_alpha=True, row_end=row_end)
+        loglike = backend.loglike_multi if multi else backend.loglike
+        _, info, alpha, ws = loglike(Xd, yd, e2, desc, want_alpha=True, row_end=row_end)
         bad = int(info.item())
         if bad < 0:
             raise _cabi.TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % bad)
@@ -219,7 +237,7 @@ class GPInterpolation(object):
             a[order], z[order] = alpha, zdiag
             alpha, zdiag = a, z
         alpha, zdiag = alpha.cpu().numpy(), zdiag.cpu().numpy()
-        mean = y - alpha / zdiag + self._mean + self._spatial_average
+        mean = y - alpha / (zdiag[:, None] if multi else zdiag) + self._mean + self._spatial_average
         return mean, 1.0 / zdiag - e2_host
 
     def return_gp_predict(self, y, X1, X2, kernel, y_err, return_cov=False):
@@ -230,7 +248,7 @@ class GPInterpolation(object):
         n = Xd.shape[0]
         Xs = backend.as_points(X2)
         m = Xs.shape[0]
-        y_predict = backend.predict_mean(Xs, Xd, desc, self._alpha_dev).cpu().numpy()
+        y_predict = self._predict_mean(Xs, Xd, desc).cpu().numpy()
         if not return_cov:
             return y_predict, None
         # y_cov = K** - K* (K + s^2 I)^-1 K*^T = K** - V V^T,  V = K* L^-T  (gp_interp.py:187-191)
@@ -244,11 +262,14 @@ class GPInterpolation(object):
         """Attach the data: positions X (n, 1|2), values y (n,), optional errors y_err (n,); looks up the
         mean function, folds in the white noise, computes the normalising mean and drops any cached
         solve (gp_interp.py:196-227)."""
+        multi = np.ndim(y) == 2
+        if multi:
+            _check_multi_inputs(y, y_err, self._has_average, self._y0, self.indice_meanify)
         self.kernel = copy.deepcopy(self.kernel_template)
         self._X = X
         self._y = y
         if y_err is None:
-            y_err = np.zeros_like(y)
+            y_err = np.zeros(len(y)) if multi else np.zeros_like(y)
         self._y_err = y_err
 
         if self._X0 is None:
@@ -261,7 +282,13 @@ class GPInterpolation(object):
         self._y_err = y_err
 
         if self.normalize:
-            self._mean = np.mean(y - self._spatial_average)
+            # several outputs: one mean per column, _mean has shape (r,); column by column, so that each output is
+            # normalised exactly as it would be on its own (numpy sums a strided axis in another order)
+            if multi:
+                res = np.asarray(y - self._spatial_average)
+                self._mean = np.array([np.mean(np.ascontiguousarray(res[:, c])) for c in range(res.shape[1])])
+            else:
+                self._mean = np.mean(y - self._spatial_average)
         else:
             self._mean = 0.0
         # alpha / L are recomputed whenever the input data change
@@ -272,17 +299,19 @@ class GPInterpolation(object):
         """Mean function at X: uniform mean of the `n_neighbors` nearest grid values of the meanify table,
         or zeros when no table was given (gp_interp.py:229-243)."""
         X = np.asarray(X)
+        multi = np.ndim(self._y) == 2
         if np.count_nonzero(self._X0) == 0:
-            return np.zeros(len(X[:, 0]))
+            return np.zeros((len(X[:, 0]), np.shape(self._y)[1])) if multi else np.zeros(len(X[:, 0]))
         from .meanify import knn_average
 
         average = knn_average(self._X0, self._y0, X, self.n_neighbors)
         if self.indice_meanify is not None:
-            average = average[:, self.indice_meanify]
+            average = average[:, list(self.indice_meanify) if multi else self.indice_meanify]
         return average
 
     def solve(self):
         """Fit the kernel hyper-parameters with the configured optimizer (gp_interp.py:245-258)."""
+        self._check_2pcf_output()
         self._init_theta = [copy.deepcopy(self.kernel).theta]
         self.kernel = self._fit(
             self.kernel,
@@ -294,6 +323,7 @@ class GPInterpolation(object):
     def return_2pcf(self):
         """xi, its weight matrix, separations, bin coordinates and mask for the current data
         (gp_interp.py:260-275)."""
+        self._check_2pcf_output(always=True)
         pcf = two_pcf(
             self._X,
             self._y - self._mean - self._spatial_average,
@@ -304,6 +334,12 @@ class GPInterpolation(object):
             anisotropic=self.optimizer == "anisotropic",
         )
         return pcf.return_2pcf()
+
+    def _check_2pcf_output(self, always=False):
+        """The 2-point correlation function fit is defined for one scalar field."""
+        if np.ndim(self._y) == 2 and (always or self.optimizer in ["two-pcf", "anisotropic"]):
+            raise ValueError("the two-pcf / anisotropic fit and return_2pcf need a 1-D y; with several outputs use "
+                             "optimizer='log-likelihood' or 'none'")
 
     def return_log_likelihood(self, theta=None):
         """Marginal log-likelihood of the current data for the current kernel, or for `theta` if given
@@ -351,3 +387,32 @@ class GPInterpolation(object):
                 plt.ylabel(r"$\Delta y$", fontsize=16)
             plt.title(title, fontsize=16)
         return fig
+
+
+def _device_outputs(y):
+    """y on the device: (n,) for one output (any shape flattened, as the reference does), (n, r) for several."""
+    y = np.asarray(y, dtype=np.float64)
+    return backend.to_device(y if y.ndim == 2 else y.reshape(-1))
+
+
+def _check_multi_inputs(y, y_err, has_average, y0, indice_meanify):
+    """Several outputs: y (n, r) with 1 <= r <= TGP_MAX_RHS, y_err None or (n,) shared by the outputs, and with a
+    meanify table r column indices (None only when the table has exactly r columns)."""
+    n, r = np.shape(y)
+    if not 1 <= r <= _cabi.MAX_RHS:
+        raise ValueError("y has %d outputs; at most %d (TGP_MAX_RHS) share one kernel" % (r, _cabi.MAX_RHS))
+    if y_err is not None and np.shape(y_err) != (n,):
+        raise ValueError("with several outputs y_err must have shape (n,) = (%d,), shared by the outputs; got %r"
+                         % (n, np.shape(y_err)))
+    if has_average:
+        ncols = np.shape(y0)[1] if np.ndim(y0) == 2 else 1
+        if indice_meanify is None:
+            if np.ndim(y0) != 2 or ncols != r:
+                raise ValueError("indice_meanify=None needs a meanify table with exactly %d columns; it has %d"
+                                 % (r, ncols))
+        else:
+            idx = np.atleast_1d(np.asarray(indice_meanify))
+            if (idx.ndim != 1 or len(idx) != r or idx.dtype.kind not in "iu" or np.ndim(y0) != 2
+                    or np.any(idx < -ncols) or np.any(idx >= ncols)):
+                raise ValueError("indice_meanify must list %d column indices of the meanify table (%d columns); got %r"
+                                 % (r, ncols, indice_meanify))

@@ -28,6 +28,9 @@ class log_likelihood(object):
 
     X: (n, 1|2) positions; y: (n,) residual field values; y_err: (n,) one-sigma errors added in quadrature
     on the diagonal.  Same constructor as the reference class of the same name.
+
+    y of shape (n, r), 1 <= r <= 8 (extension): r outputs sharing the kernel and y_err.  The log-likelihood is then the
+    joint value sum_c logL_c (scikit-learn's log_marginal_likelihood for multi-target y), from one factorisation.
     """
 
     def __init__(self, X, y, y_err):
@@ -41,9 +44,14 @@ class log_likelihood(object):
     def _device_state(self):
         if self._dev is None:
             Xd = backend.as_points(self.X)
-            yd = backend.to_device(np.asarray(self.y, dtype=np.float64).reshape(-1))
+            if np.ndim(self.y) == 2:   # several outputs: r extra rows ride through potrf
+                yd = backend.to_device(np.asarray(self.y, dtype=np.float64))
+                rows = yd.shape[1]
+            else:
+                yd = backend.to_device(np.asarray(self.y, dtype=np.float64).reshape(-1))
+                rows = 1
             e2 = backend.to_device(np.asarray(self.y_err, dtype=np.float64).reshape(-1) ** 2)
-            work = backend.alloc_matrix(self.ndata + 1, self.ndata, Xd.device)  # +1 row: y rides through potrf
+            work = backend.alloc_matrix(self.ndata + rows, self.ndata, Xd.device)  # the outputs ride through potrf
             self._dev = (Xd, yd, e2, work)
             self._sorted_axes = {}   # backend.plan_envelope's cache: order / coordinates per sorting axis
             self._sorted_data = {}   # axis -> (X, y, y_err^2) in that order
@@ -76,11 +84,12 @@ class log_likelihood(object):
         if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf
         banded = self._envelope_inputs(desc)
+        loglike = backend.loglike_multi if yd.dim() == 2 else backend.loglike
         if banded is None:
-            out, info, _, _ = backend.loglike(Xd, yd, e2, desc, work=work, want_alpha=False)
+            out, info, _, _ = loglike(Xd, yd, e2, desc, work=work, want_alpha=False)
         else:
-            out, info, _, _ = backend.loglike(banded[0], banded[1], banded[2], desc, work=work, want_alpha=False,
-                                              row_end=banded[3])
+            out, info, _, _ = loglike(banded[0], banded[1], banded[2], desc, work=work, want_alpha=False,
+                                      row_end=banded[3])
             self.n_banded_evaluations = getattr(self, "n_banded_evaluations", 0) + 1
         self.n_evaluations += 1
         value = float(out[0].item())  # -inf when the matrix is not positive definite (info > 0)
@@ -102,10 +111,12 @@ class log_likelihood(object):
         if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf, np.zeros(J.shape[1])
         banded = self._envelope_inputs(desc)
+        # several outputs: tgp_loglike_grad_multi, whose out has the sum layout (a single term's four derivatives first)
+        loglike_grad = backend.loglike_grad_multi if yd.dim() == 2 else backend.loglike_grad
         if banded is None:
-            out, info, _, _ = backend.loglike_grad(Xd, yd, e2, desc, work=work)
+            out, info, _, _ = loglike_grad(Xd, yd, e2, desc, work=work)
         else:
-            out, info, _, _ = backend.loglike_grad(banded[0], banded[1], banded[2], desc, work=work, row_end=banded[3])
+            out, info, _, _ = loglike_grad(banded[0], banded[1], banded[2], desc, work=work, row_end=banded[3])
             self.n_banded_evaluations = getattr(self, "n_banded_evaluations", 0) + 1
         self.n_evaluations += 1
         o = out.cpu().numpy()
