@@ -306,16 +306,22 @@ typedef enum {
  * Outputs are ACCUMULATED into (the caller zeroes them).  xi = sumwkk / sumw is left to the caller
  * so that multi-GPU partial sums can be all-reduced first.
  *  work           : optional 32-byte aligned device scratch of tgp_pairbin_work_doubles(total, ncat)
- *                   doubles (bounding boxes of the 32-point chunks, filled by a pre-pass).  NULL: the
- *                   boxes are recomputed on the fly (slower when most blocks are out of range).
- */
+ *                   doubles (bounding boxes, sums and sorted copies of the 32-point chunks, filled by a
+ *                   pre-pass; for TwoD also the block records and work counters of the two-pass count, see
+ *                   below).  NULL: no block forms (TwoD: pair by pair; Log: the boxes are recomputed on the fly);
+ *                   the counts are the same.
+ * TwoD with work runs in rounds of this rank's items: a classification pass books the blocks that sit in one
+ * bin and records the others, then a second kernel processes the recorded blocks.  A round holds at most
+ * 2^26 records (1 GiB of `work` at N >= ~4e5; fewer for smaller catalogues), about 8 rounds at N = 1e6. */
 int tgp_pairbin(const double* px, const double* py, const double* pk, const double* pw,
                 const int64_t* cat_off, int32_t ncat, int64_t max_cat_len, int32_t bin_type,
                 const double* edges, int32_t nbins, double min_sep2, double max_sep,
                 int32_t tile_rank, int32_t tile_nranks, int64_t* npairs, double* sumw,
                 double* sumwkk, double* sumwr, double* work, void* stream);
 
-/* Size (in doubles) of the optional scratch buffer of tgp_pairbin. */
+/* Size (in doubles) of the optional scratch buffer of tgp_pairbin for catalogues of `total_points` points in
+ * all (an upper bound on max_cat_len is enough): the chunk records of the pre-pass plus the block records of one
+ * round, capped at 2^26 records of 16 bytes. */
 int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat);
 
 /* Hilbert-curve keys of 2-D points on a 2^order x 2^order grid over the square
@@ -427,7 +433,8 @@ int tgp_device_error(int reset);
 int tgp_pairbin_tile(void);
 
 /* Diagnostics: how many pairs (32 x columns per processed block) of all tgp_pairbin launches since the last
- * reset went through each path: host8[0] closed form (whole block in one bin and its mirror image), [1] one
+ * reset went through each path: host8[0] closed form (whole block in one bin and its mirror image; TwoD: booked by
+ * the classification pass, the other slots by the pass over the recorded blocks), [1] one
  * varying axis (one compare pair per pair of points), [2] pair by pair in a 2 x 2 bin window or through the
  * generic path (the diagonal blocks are not tallied), [3] one varying axis answered by a rank query on the
  * chunk's sorted copy (8 probes per row point instead of 32 compares), [4] 2 x 2 bin window with the column-bit
@@ -441,7 +448,8 @@ int tgp_pairbin_stats(unsigned long long* host8 /*host*/, int reset);
  * "pairbin_fast_paths": bit mask, default all on; bit 0 = short-cut dispatch of one-axis blocks that fit the open
  * bin window, bit 1 = 2 x 2-window blocks take their marginal sums from rank queries, bit 2 = the pair-by-pair kernel
  * ("pairbin_block_sums" 0) skips the per-pair mirrored-bin check in blocks whose bounding boxes prove it
- * (0 = the general paths only; results are identical either way); "bootbin_paths": bit mask of tgp_bootbin_twod,
+ * (0 = the general paths only; results are identical either way); "pairbin_record_cap": block records per round of
+ * the two-pass TwoD count, at least 256, at most (and <= 0: back to) the default 2^26 -- more, smaller rounds; "bootbin_paths": bit mask of tgp_bootbin_twod,
  * default all on; bit 0 = blocks in one bin booked from chunk sums, bit 1 = window paths (0: every block through the
  * exact per-pair path), bit 2 = axis sweeps, bit 3 = blocks spanning more than 2 x 2 bins summed bin by bin. */
 int tgp_set_option(const char* name, int value);

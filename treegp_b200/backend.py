@@ -625,7 +625,8 @@ _PB_SCRATCH = {}
 
 
 def _pairbin_scratch(dev, doubles):
-    """The pre-pass workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6), kept per
+    """The workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6, plus the block records of
+    one round of the two-pass TwoD count, at most 1 GiB), kept per
     (device, stream) and grown on demand: launches on one stream are ordered, so they can share it; launches on
     different streams get different buffers."""
     key = (dev.index, torch.cuda.current_stream(dev).cuda_stream)

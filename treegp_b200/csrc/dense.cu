@@ -201,6 +201,7 @@ static int gemm_nt_sub_launch(double* C, int64_t M, int64_t Nc, int64_t ldc, con
 
 extern "C" int tgp_pairbin_set_block_sums(int on);
 extern "C" int tgp_pairbin_set_fast_paths(int bits);
+extern "C" int tgp_pairbin_set_record_cap(int n);
 extern "C" int tgp_trsv_set_cluster(int v);
 extern "C" int tgp_bootbin_set_paths(int bits);
 extern "C" int tgp_set_option(const char* name, int value) {
@@ -211,6 +212,7 @@ extern "C" int tgp_set_option(const char* name, int value) {
   if (name && !strcmp(name, "potrf_env_lookahead")) { g_env_lookahead = value; return TGP_OK; }
   if (name && !strcmp(name, "pairbin_block_sums")) return tgp_pairbin_set_block_sums(value);
   if (name && !strcmp(name, "pairbin_fast_paths")) return tgp_pairbin_set_fast_paths(value);
+  if (name && !strcmp(name, "pairbin_record_cap")) return tgp_pairbin_set_record_cap(value);
   if (name && !strcmp(name, "bootbin_paths")) return tgp_bootbin_set_paths(value);
   if (name && !strcmp(name, "potrf_ob") && value >= 0 && value % 512 == 0) { g_ob_large = value; return TGP_OK; }
   tgp_set_error("tgp_set_option: unknown option");

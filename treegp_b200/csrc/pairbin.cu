@@ -22,12 +22,17 @@
 // registers; the warp stages one column chunk at a time in its private slice of shared memory and
 // reads it back as broadcasts.
 //
+// TwoD with block forms runs as TWO kernels per round of items (tgp_pairbin): pairbin_classify_kernel classifies every
+// block from the chunk boxes, books the closed-form blocks and records the others; pairbin_kernel<TwoD, W, true> then
+// runs the paths below over the recorded blocks only.  The classification needs none of the per-row register state
+// of the residual paths, so it runs at more warps per SM and the residual kernel's warm code no longer contains it.
+//
 // Two instantiations per bin type (template parameter BS):
 //   BS = false  the pair-by-pair kernel: every pair of every in-range block is evaluated individually
 //               (tgp_set_option("pairbin_block_sums", 0)); the 10-FP64-ops-per-pair roofline is stated for it.
 //               Blocks that provably sit in one bin per axis whose mirrored window is the mirror image skip the
 //               per-pair mirrored bits (the forward bits are still evaluated for every pair).
-//   BS = true   (default) block forms on top of the same classification, all exact:
+//   BS = true   (default) block forms on top of the same classification, all exact (TwoD: pass B, see above):
 //               * TwoD, block in ONE forward bin whose mirrored window is its mirror image: booked whole by the
 //                 classifying lane from the chunk sums of the pre-pass (points never loaded);
 //               * TwoD, one varying axis: rank query (4-ary search, 8 probes per row point) on the chunk's copy
@@ -84,9 +89,17 @@ struct PBParams {
   int32_t fast_paths;     // bit 0: short-cut dispatch of one-axis blocks that fit the open window; bit 1: 2 x 2-window
                           // blocks with marginal sums from rank queries; bit 2: pair-by-pair kernel, no mirrored bits
                           // per pair in blocks that provably sit in one bin and its mirror image (default: all)
+  // TwoD block forms, two passes per round (pairbin_classify_kernel, then pairbin_kernel<TwoD, W, true>): this
+  // round's items q in [q_begin, q_end) of this rank; the records of item q at recs + (q - q_begin) * run, their
+  // number at rec_cnt[q - q_begin]; counter_next = the other pass's work counter, zeroed for its next launch
+  int64_t q_begin, q_end;
+  int4* recs;
+  int* rec_cnt;
+  unsigned long long* counter_next;
 };
 
-// Which path the pairs of all launches since the last reset took (in pairs): [0] closed form (block in one bin),
+// Which path the pairs of all launches since the last reset took (in pairs): [0] closed form (block in one bin; TwoD:
+// tallied by the classification pass, the others by the pass over the recorded blocks),
 // [1] one varying axis, pair by pair, [2] pair by pair (2 x 2 window with or without the per-pair range test,
 // generic sub-blocks), [3] one varying axis answered by a rank query on the sorted chunk, [4] 2 x 2 window with the
 // marginal sums from rank queries (one quadrant pair by pair).  Diagnostics.
@@ -445,7 +458,9 @@ enum { PB_OUT = 0, PB_REG_FULL = 1, PB_REG_CHECK = 2, PB_GENERIC = 3 };
 
 // Classification of one (row block, column block) pair from the two bounding boxes.
 // Returns the class; for REG classes w[0..3] receive the packed windows (origin | extent << 16) of the
-// forward x, forward y, mirrored x and mirrored y bins.
+// forward x, forward y, mirrored x and mirrored y bins.  INLINE_SEARCH: the rare fallback search of the mirrored ends
+// is inlined instead of called (no call, so no registers saved around it: the small classification kernel).
+template <bool INLINE_SEARCH = false>
 __device__ __forceinline__ int pb_classify_twod(double iminx, double imaxx, double iminy, double imaxy,
                                                 double cminx, double cmaxx, double cminy, double cmaxy,
                                                 double M, double lo2, int nbins, const double* __restrict__ ed,
@@ -463,8 +478,12 @@ __device__ __forceinline__ int pb_classify_twod(double iminx, double imaxx, doub
   const int y0 = pb_bin_twod_search(dy0, nbins, ed), y1 = pb_bin_twod_search(dy1, nbins, ed);
   // mirrored ends: the grid is point symmetric up to rounding of the thresholds, so bin(-d) is nbins-1-bin(d)
   // unless d sits within a few ulp of an edge; the guess is verified against the thresholds (exact either way)
-  const int rx0 = pb_bin_twod_guess(-dx1, nbins - 1 - x1, nbins, ed), rx1 = pb_bin_twod_guess(-dx0, nbins - 1 - x0, nbins, ed);
-  const int ry0 = pb_bin_twod_guess(-dy1, nbins - 1 - y1, nbins, ed), ry1 = pb_bin_twod_guess(-dy0, nbins - 1 - y0, nbins, ed);
+  auto guess = [&](double d, int g) {
+    if (INLINE_SEARCH) return (d >= ed[g] && d < ed[g + 1]) ? g : pb_bin_twod_search(d, nbins, ed);
+    return pb_bin_twod_guess(d, g, nbins, ed);
+  };
+  const int rx0 = guess(-dx1, nbins - 1 - x1), rx1 = guess(-dx0, nbins - 1 - x0);
+  const int ry0 = guess(-dy1, nbins - 1 - y1), ry1 = guess(-dy0, nbins - 1 - y0);
   if (x1 - x0 > 1 || y1 - y0 > 1 || rx1 - rx0 > 1 || ry1 - ry0 > 1) return PB_GENERIC;
   w[0] = x0 | ((x1 - x0) << 16);
   w[1] = y0 | ((y1 - y0) << 16);
@@ -472,6 +491,54 @@ __device__ __forceinline__ int pb_classify_twod(double iminx, double imaxx, doub
   w[3] = ry0 | ((ry1 - ry0) << 16);
   return (ax < M && ay < M && r2min >= lo2) ? PB_REG_FULL : PB_REG_CHECK;
 }
+
+// Work item q of this rank -> catalogue, row block ib and column chunks [c_lo, c_hi).  Returns false for an empty
+// item (past the end of a shorter catalogue); stop = true once q is past the last catalogue.  pairbin_kernel keeps
+// the same decode inline: calling this helper there changes the register allocation of its pair-by-pair and Log
+// instantiations, whose code is the reference the timings are stated for.
+struct PBItem {
+  int cat;
+  int64_t off, n, ib, c_lo, c_hi;
+};
+__device__ __forceinline__ bool pb_decode_item(const PBParams& P, int64_t q, PBItem& it, bool& stop) {
+  const int64_t item = q * P.nranks + P.rank;
+  const int R = P.run;
+  const int cat = (int)(item / P.items_per_cat);
+  stop = cat >= P.ncat;
+  if (stop) return false;
+  const int64_t lq = item % P.items_per_cat;
+  const int64_t off = P.cat_off[cat];
+  const int64_t n = P.cat_off[cat + 1] - off;
+  const int64_t nblk = (n + PB_CHUNK - 1) / PB_CHUNK;
+  if (nblk == 0) return false;
+  const int64_t nruns = (nblk + R - 1) / R;
+  // decode lq -> (row block ib, run r): rows of group g = ib / R pair with runs g .. nruns-1;
+  // items before group g: R * (g*nruns - g*(g-1)/2)
+  const double tn = 2.0 * (double)nruns + 1.0;
+  const double disc = tn * tn - 8.0 * (double)lq / (double)R;
+  int64_t g = (int64_t)((tn - sqrt(disc > 0.0 ? disc : 0.0)) * 0.5);
+  if (g < 0) g = 0;
+  if (g >= nruns) g = nruns - 1;
+  while (g > 0 && (int64_t)R * (g * nruns - g * (g - 1) / 2) > lq) --g;
+  while (g + 1 < nruns && (int64_t)R * ((g + 1) * nruns - (g + 1) * g / 2) <= lq) ++g;
+  const int64_t rem = lq - (int64_t)R * (g * nruns - g * (g - 1) / 2);
+  const int64_t per_row = nruns - g;
+  const int64_t row_in_g = rem / per_row;
+  const int64_t ib = g * R + row_in_g;
+  const int64_t r = g + rem % per_row;
+  if (row_in_g >= R || ib >= nblk) return false;  // past the end of this (shorter) catalogue
+  it.cat = cat;
+  it.off = off;
+  it.n = n;
+  it.ib = ib;
+  it.c_lo = (r * R > ib) ? r * R : ib;
+  it.c_hi = ((r + 1) * R < nblk) ? (r + 1) * R : nblk;
+  return it.c_lo < it.c_hi;
+}
+
+// A window of pb_classify_twod (origin < 4096 | extent <= 1 << 16) in the 13 bits of a record field, and back.
+__device__ __forceinline__ int pb_pack_win(int w) { return (w & 0xfff) | ((w >> 16) << 12); }
+__device__ __forceinline__ int pb_unpack_win(int v) { return (v & 0xfff) | (((v >> 12) & 1) << 16); }
 
 #ifndef PB_MIN_CTAS
 #define PB_MIN_CTAS 2
@@ -482,6 +549,8 @@ __device__ __forceinline__ int pb_classify_twod(double iminx, double imaxx, doub
 template <int BT, bool WEIGHTED, bool BS>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_MIN_CTAS)
 pairbin_kernel(PBParams P) {
+  // TwoD with block forms is pass B of the two-pass count: the blocks come from the records of pass A
+  constexpr bool PASS_B = BS && BT == TGP_BIN_TWOD;
   extern __shared__ __align__(16) unsigned char pb_smem[];
   const int nb = P.nb, nbins = P.nbins, nwarps = P.warps;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -510,6 +579,9 @@ pairbin_kernel(PBParams P) {
     if (BT == TGP_BIN_LOG) my_r[i] = 0.0;
   }
   __syncthreads();  // the only CTA-wide barrier
+  if constexpr (PASS_B) {
+    if (blockIdx.x == 0 && tid == 0) *P.counter_next = 0ull;   // pass A of the next round starts from zero
+  }
 
   RegAcc<WEIGHTED> A;
   A.zero();
@@ -678,20 +750,6 @@ pairbin_kernel(PBParams P) {
     return !live || ((pos == 0 || cxy[pos - 1].x <= RT) && (pos == PB_CHUNK || cxy[pos].x > RT));
   };
 
-  // per-lane open bin of the blocks booked whole at classification time (forward bin cf_bin and its mirror image)
-  int cf_bin = -1;
-  unsigned cf_cnt = 0u;
-  double cf_s = 0.0, cf_w = 0.0;
-  auto cf_spill = [&]() {
-    if (cf_bin >= 0 && cf_cnt) {
-      atomicAdd(my_c + cf_bin, cf_cnt);    // forward entry; the mirror image is added by flush_hist
-      atomicAdd(my_s + cf_bin, cf_s);
-      if constexpr (WEIGHTED) atomicAdd(my_w + cf_bin, cf_w);
-    }
-    cf_cnt = 0u;
-    cf_s = 0.0;
-    cf_w = 0.0;
-  };
   const double M = P.hi, lo2 = P.lo2;
   const int R = P.run;
   unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0;   // column counts (x 32 rows = pairs) per path
@@ -699,9 +757,18 @@ pairbin_kernel(PBParams P) {
   while (true) {
     // ---- next work item for this warp ----
     unsigned long long q = 0;
-    if (lane == 0) q = atomicAdd(P.counter, 1ull);
-    q = __shfl_sync(0xffffffffu, q, 0);
-    if ((int64_t)q >= P.my_items) break;
+    int nrec = 0;
+    if constexpr (PASS_B) {
+      if (lane == 0) q = atomicAdd(P.counter, 1ull);
+      q = __shfl_sync(0xffffffffu, q, 0) + (unsigned long long)P.q_begin;
+      if ((int64_t)q >= P.q_end) break;
+      nrec = P.rec_cnt[q - P.q_begin];
+      if (nrec == 0) continue;
+    } else {
+      if (lane == 0) q = atomicAdd(P.counter, 1ull);
+      q = __shfl_sync(0xffffffffu, q, 0);
+      if ((int64_t)q >= P.my_items) break;
+    }
     const int64_t item = (int64_t)q * P.nranks + P.rank;
     const int cat = (int)(item / P.items_per_cat);
     if (cat >= P.ncat) break;
@@ -751,14 +818,17 @@ pairbin_kernel(PBParams P) {
     const long long owner = (long long)(off + ib * PB_CHUNK);
     // pre-pass record of chunk c of this catalogue: slot (off + 32 c) / 32 + cat = off / 32 + c + cat
     const double* rec0 = P.boxes ? P.boxes + (size_t)PB_STRIDE * (size_t)(off / PB_CHUNK + cat) : nullptr;
-    // row-block aggregates for the blocks that are booked whole
+    // row-block aggregates for the Log blocks that are booked whole
     const double rowK = warp_sum(ki);
     double rowW = 0.0;
     if constexpr (WEIGHTED) rowW = warp_sum(wi);
     const int nlive = __popc(__ballot_sync(0xffffffffu, live));
+    // pass B: the records of this item, in chunk order
+    const int4* irec = PASS_B ? P.recs + (size_t)(q - P.q_begin) * (size_t)P.run : nullptr;
 
-    for (int64_t sc = c_lo; sc < c_hi; sc += 32) {
-      // ---- lane l classifies column chunk sc + l ----
+    // pass B walks the item's records, 32 at a time; otherwise 32 column chunks at a time
+    for (int64_t sc = PASS_B ? 0 : c_lo; sc < (PASS_B ? (int64_t)nrec : c_hi); sc += 32) {
+      // ---- lane l classifies column chunk sc + l (pass B: loads record sc + l) ----
       const int64_t mychunk = sc + lane;
       int cls = PB_OUT;
       int kind = 0;   // 0: raw points; 1 / 2: one-axis block answered from the x- / y-sorted copy of the chunk
@@ -767,7 +837,20 @@ pairbin_kernel(PBParams P) {
       // open window covers the block; 0 otherwise
       int fastw = 0;
       int win[4] = {0, 0, 0, 0};
-      if (mychunk < c_hi) {
+      int roff = 0;   // pass B: the record's chunk, relative to c_lo
+      if (PASS_B) {
+        if (mychunk < nrec) {
+          const int4 rr = irec[mychunk];
+          roff = rr.x & 0xff;
+          cls = (rr.x >> 8) & 3;
+          kind = (rr.x >> 10) & 3;
+          fastw = rr.y;
+          win[0] = pb_unpack_win(rr.z);
+          win[1] = pb_unpack_win(rr.z >> 16);
+          win[2] = pb_unpack_win(rr.w);
+          win[3] = pb_unpack_win(rr.w >> 16);
+        }
+      } else if (mychunk < c_hi) {
         const int64_t j0g = mychunk * PB_CHUNK;
         const int cnt = (int)((n - j0g < PB_CHUNK) ? (n - j0g) : PB_CHUNK);
         double cminx = INFINITY, cmaxx = -INFINITY, cminy = INFINITY, cmaxy = -INFINITY;
@@ -808,36 +891,6 @@ pairbin_kernel(PBParams P) {
           if (mychunk == ib) cls = PB_GENERIC;
         }
         if (!(iminx <= imaxx)) cls = PB_OUT;  // no live row in this warp
-        if (BS && BT == TGP_BIN_TWOD && cls == PB_REG_FULL && P.boxes) {
-          // Whole block in ONE forward bin and in its mirror image: the classifying lane books the block itself
-          // from the chunk sums of the pre-pass (count = rows x columns, sum = (sum of the rows' k w) x (sum of the
-          // columns' k w)); the points of the chunk are never loaded.  Consecutive chunks of a lane mostly hit
-          // the same bin: the lane keeps one open bin in registers and spills to the warp histogram on a change.
-          const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
-          const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
-          const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
-          // exactly one varying axis: the block is answered from the chunk's points sorted along that axis
-          if (P.sorted && cnt == PB_CHUNK) kind = (one_y && !one_x) ? 1 : ((one_x && !one_y) ? 2 : 0);
-          if (P.fast_paths & 1) {
-            const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
-            const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
-            if ((kind == 1 && clean_x) || (kind == 2 && clean_y)) fastw = 1 | (kind << 1) | (x0 << 3) | (y0 << 15);
-          }
-          // two bins along BOTH axes: the raw points are staged as usual (kind stays 0); field value 3
-          if ((P.fast_paths & 2) && P.sorted && cnt == PB_CHUNK && (win[0] >> 16) == 1 && (win[2] >> 16) == 1 &&
-              rx0 == nbins - 2 - x0 && (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0)
-            fastw = 1 | (3 << 1) | (x0 << 3) | (y0 << 15);
-          if (one_x && one_y) {
-            const double2 sums = *reinterpret_cast<const double2*>(rec0 + (size_t)PB_STRIDE * (size_t)mychunk + 4);
-            const int o = y0 * nbins + x0;
-            if (o != cf_bin) { cf_spill(); cf_bin = o; }
-            cf_cnt += (unsigned)(nlive * cnt);
-            cf_s = fma(rowK, sums.x, cf_s);
-            if constexpr (WEIGHTED) cf_w = fma(rowW, sums.y, cf_w);
-            st_closed += (unsigned)cnt;
-            cls = PB_OUT;
-          }
-        }
       }
       const unsigned todo = __ballot_sync(0xffffffffu, cls != PB_OUT);
       // ---- process the non-OUT chunks; the next chunk's points are prefetched into registers ----
@@ -845,8 +898,13 @@ pairbin_kernel(PBParams P) {
       double nx_ = 0.0, ny_ = 0.0, nk_ = 0.0, nw_ = 1.0;
       double2 nsum_ = make_double2(0.0, 0.0);
       int nkind_ = 0;
+      // the column chunk of lane c's block
+      auto chunk_of = [&](int c) -> int64_t {
+        if constexpr (PASS_B) return c_lo + __shfl_sync(0xffffffffu, roff, c);
+        else return sc + c;
+      };
       auto fetch_raw = [&](int c) {
-        const int64_t jg = (sc + c) * PB_CHUNK + lane;
+        const int64_t jg = chunk_of(c) * PB_CHUNK + lane;
         const bool ok = jg < n;
         nx_ = ok ? P.px[off + jg] : 0.0;
         ny_ = ok ? P.py[off + jg] : 0.0;
@@ -854,7 +912,7 @@ pairbin_kernel(PBParams P) {
         nk_ = ok ? P.pk[off + jg] * nw_ : 0.0;
       };
       auto fetch = [&](int c) {
-        const double* rec = rec0 + (size_t)PB_STRIDE * (size_t)(sc + c);
+        const double* rec = rec0 + (size_t)PB_STRIDE * (size_t)chunk_of(c);
         if (P.boxes) nsum_ = *reinterpret_cast<const double2*>(rec + 4);   // chunk sums of k w and w (pre-pass)
         if constexpr (!BS) {
           fetch_raw(c);
@@ -909,7 +967,7 @@ pairbin_kernel(PBParams P) {
               // row-bit sums are rank queries on the x- / y-sorted copies (read from global memory: their lines
               // are pulled in while the pair loop runs); only the "both bits" quadrant is summed pair by pair.
               if (bx0 == A.fx0 && by0 == A.fy0) {
-                const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)(sc + c) + PB_SLOT;
+                const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)chunk_of(c) + PB_SLOT;
                 const double* srty = srt + 3 * PB_CHUNK;
                 const double x7 = srt[7], x15 = srt[15], x23 = srt[23];
                 const double y7 = srty[7], y15 = srty[15], y23 = srty[23];
@@ -984,13 +1042,13 @@ pairbin_kernel(PBParams P) {
             }
           }
         }
-        const int64_t j0g = (sc + c) * PB_CHUNK;
+        const int64_t j0g = chunk_of(c) * PB_CHUNK;
         const int jcount = (int)((n - j0g < PB_CHUNK) ? (n - j0g) : PB_CHUNK);
         int ccls = __shfl_sync(0xffffffffu, cls, c);
         // Log bins and the diagonal block (needs j > i) go pair by pair through the generic path -- which has ONE
         // call site, at the top of the sub-block loop below, so that its code exists once in the kernel
-        const bool whole_generic = (BT != TGP_BIN_TWOD && ccls == PB_GENERIC) || (sc + c) == ib;
-        const int gfirst = ((sc + c) == ib) ? lane + 1 : 0;
+        const bool whole_generic = (BT != TGP_BIN_TWOD && ccls == PB_GENERIC) || chunk_of(c) == ib;
+        const int gfirst = (chunk_of(c) == ib) ? lane + 1 : 0;
         int cw4[4];
 #pragma unroll
         for (int k = 0; k < 4; ++k) cw4[k] = __shfl_sync(0xffffffffu, win[k], c);
@@ -1306,8 +1364,6 @@ pairbin_kernel(PBParams P) {
       }
     }
     // bound the per-lane 32-bit counters: registers go to shared memory at the end of every item
-    cf_spill();
-    cf_bin = -1;
     __syncwarp();
     flush_regs();
   }
@@ -1321,6 +1377,169 @@ pairbin_kernel(PBParams P) {
     if (st_sorted) atomicAdd(&g_pb_stats[3], 32ull * st_sorted);
     if (st_quad) atomicAdd(&g_pb_stats[4], 32ull * st_quad);
   }
+}
+
+// Pass A of the TwoD block forms: classify and book.  Same items and dealing as pairbin_kernel; a warp takes an item
+// of this round, reads the row block's box, sums and live count from the pre-pass record of chunk ib (no point is
+// loaded), and lane l classifies chunk sc + l from the boxes exactly as the fused kernel did:
+//   * a block in ONE forward bin whose mirrored window is its mirror image is booked whole from the chunk sums
+//     (count = rows x columns, sum = (rows' sum of k w) x (columns' sum of k w)); consecutive chunks of a lane mostly hit
+//     the same bin, so the lane keeps one open bin in registers and spills to the warp histogram on a change;
+//   * every other block that is not OUT (the diagonal block as GENERIC) is appended to the item's records in chunk
+//     order: {chunk - c_lo | class << 8 | kind << 10, fastw, packed forward windows, packed mirrored windows}.
+// kind 1 / 2: one varying axis, answered from the x- / y-sorted copy of the chunk; fastw != 0: the block may take
+// one of pass B's short cuts (see there).  The warp histograms hold forward entries; the mirror image is added
+// when they are written out.
+#ifndef PB_CLASSIFY_MIN_CTAS
+#define PB_CLASSIFY_MIN_CTAS 2
+#endif
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_CLASSIFY_MIN_CTAS)
+pairbin_classify_kernel(PBParams P) {
+  extern __shared__ __align__(16) unsigned char pb_smem[];
+  const int nb = P.nb, nbins = P.nbins;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  double* ed = reinterpret_cast<double*>(pb_smem);                        // nbins + 1 (padded to even)
+  double* hs_all = ed + ((nbins + 2) & ~1);                               // [warps][nb]  sum wk wk
+  double* hw_all = hs_all + (size_t)P.warps * nb;                         // [warps][nb]  sum w w     (WEIGHTED)
+  unsigned* hc_all = reinterpret_cast<unsigned*>(hw_all + (WEIGHTED ? (size_t)P.warps * nb : 0));
+  double* my_s = hs_all + (size_t)warp * nb;
+  double* my_w = hw_all + (size_t)warp * nb;
+  unsigned* my_c = hc_all + (size_t)warp * nb;
+  for (int i = tid; i <= nbins; i += blockDim.x) ed[i] = P.edges[i];
+  for (int i = lane; i < nb; i += 32) {
+    my_s[i] = 0.0;
+    my_c[i] = 0u;
+    if constexpr (WEIGHTED) my_w[i] = 0.0;
+  }
+  __syncthreads();
+  if (blockIdx.x == 0 && tid == 0) *P.counter_next = 0ull;   // pass B of this round starts from zero
+
+  auto flush_hist = [&](int cat) {   // forward entries of bin b + those of its mirror image, then clear
+    __syncwarp();
+    if (cat >= 0) {
+      for (int b = lane; b < nb; b += 32) {
+        const int bm = nb - 1 - b;
+        const unsigned long long c = (unsigned long long)my_c[b] + (unsigned long long)my_c[bm];
+        if (c) {
+          const size_t o = (size_t)cat * nb + b;
+          atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + o, c);
+          atomicAdd(P.sumwkk + o, my_s[b] + my_s[bm]);
+          atomicAdd(P.sumw + o, WEIGHTED ? my_w[b] + my_w[bm] : (double)c);
+        }
+      }
+      __syncwarp();
+      for (int b = lane; b < nb; b += 32) {
+        my_c[b] = 0u;
+        my_s[b] = 0.0;
+        if constexpr (WEIGHTED) my_w[b] = 0.0;
+      }
+    }
+    __syncwarp();
+  };
+  int cf_bin = -1;   // this lane's open bin (forward entry)
+  unsigned cf_cnt = 0u;
+  double cf_s = 0.0, cf_w = 0.0;
+  auto cf_spill = [&]() {
+    if (cf_bin >= 0 && cf_cnt) {
+      atomicAdd(my_c + cf_bin, cf_cnt);
+      atomicAdd(my_s + cf_bin, cf_s);
+      if constexpr (WEIGHTED) atomicAdd(my_w + cf_bin, cf_w);
+    }
+    cf_cnt = 0u;
+    cf_s = 0.0;
+    cf_w = 0.0;
+  };
+
+  const double M = P.hi, lo2 = P.lo2;
+  unsigned st_closed = 0;
+  int cur_cat = -1, since_flush = 0;
+  while (true) {
+    unsigned long long q = 0;
+    if (lane == 0) q = atomicAdd(P.counter, 1ull);
+    q = __shfl_sync(0xffffffffu, q, 0) + (unsigned long long)P.q_begin;
+    if ((int64_t)q >= P.q_end) break;
+    PBItem it;
+    bool stop;
+    int nrec = 0;
+    if (pb_decode_item(P, (int64_t)q, it, stop)) {
+      if (it.cat != cur_cat || since_flush >= PB_FLUSH_ITEMS) {
+        flush_hist(cur_cat);
+        cur_cat = it.cat;
+        since_flush = 0;
+      }
+      ++since_flush;
+      // 32-bit offsets from c_lo keep the register count low: the item spans <= 256 chunks, only the catalogue's last
+      // chunk can be short, and the diagonal block is the first one when c_lo == ib
+      const int64_t nblk = (it.n + PB_CHUNK - 1) / PB_CHUNK;
+      const int span = (int)(it.c_hi - it.c_lo);
+      const int tail = (int)(it.n - (nblk - 1) * PB_CHUNK);                    // points of the last chunk
+      const int last = (nblk - 1 - it.c_lo < span) ? (int)(nblk - 1 - it.c_lo) : span;
+      const bool diag = it.c_lo == it.ib;
+      const double* rec0 = P.boxes + (size_t)PB_STRIDE * (size_t)(it.off / PB_CHUNK + it.cat);
+      const double* recl = rec0 + (size_t)PB_STRIDE * (size_t)it.c_lo;
+      // the row block is chunk ib: its box and sums are the pre-pass record (the same warp reductions)
+      const double4 rb = *reinterpret_cast<const double4*>(rec0 + (size_t)PB_STRIDE * (size_t)it.ib);
+      const double2 rsum = *reinterpret_cast<const double2*>(rec0 + (size_t)PB_STRIDE * (size_t)it.ib + 4);
+      const int nlive = (it.ib == nblk - 1) ? tail : PB_CHUNK;
+      int4* out = P.recs + (size_t)(q - P.q_begin) * (size_t)P.run;
+      for (int s0 = 0; s0 < span; s0 += 32) {
+        const int ch = s0 + lane;   // chunk c_lo + ch
+        int cls = PB_OUT, kind = 0, fastw = 0;
+        int win[4] = {0, 0, 0, 0};
+        if (ch < span) {
+          const double* rec = recl + (size_t)PB_STRIDE * (size_t)ch;
+          const int cnt = (ch == last) ? tail : PB_CHUNK;
+          const double4 bb = *reinterpret_cast<const double4*>(rec);
+          if (diag && ch == 0) cls = PB_GENERIC;  // diagonal block: needs j > i
+          else cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, bb.x, bb.y, bb.z, bb.w, M, lo2, nbins, ed, win);
+          if (cls == PB_REG_FULL) {
+            const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
+            const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
+            const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
+            // exactly one varying axis: the block is answered from the chunk's points sorted along that axis
+            if (cnt == PB_CHUNK) kind = (one_y && !one_x) ? 1 : ((one_x && !one_y) ? 2 : 0);
+            // kind != 0 and the varying axis spans exactly two forward bins [v0, v0+1] whose mirrored window is the
+            // mirror image (the usual case): 1 | kind << 1 | x0 << 3 | y0 << 15, everything pass B needs to see
+            // whether its open window covers the block
+            if (P.fast_paths & 1) {
+              const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
+              const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
+              if ((kind == 1 && clean_x) || (kind == 2 && clean_y)) fastw = 1 | (kind << 1) | (x0 << 3) | (y0 << 15);
+            }
+            // two bins along BOTH axes: the raw points are staged (kind stays 0); field value 3
+            if ((P.fast_paths & 2) && cnt == PB_CHUNK && (win[0] >> 16) == 1 && (win[2] >> 16) == 1 &&
+                rx0 == nbins - 2 - x0 && (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0)
+              fastw = 1 | (3 << 1) | (x0 << 3) | (y0 << 15);
+            if (one_x && one_y) {
+              const double2 sums = *reinterpret_cast<const double2*>(rec + 4);
+              const int o = y0 * nbins + x0;
+              if (o != cf_bin) { cf_spill(); cf_bin = o; }
+              cf_cnt += (unsigned)(nlive * cnt);
+              cf_s = fma(rsum.x, sums.x, cf_s);
+              if constexpr (WEIGHTED) cf_w = fma(rsum.y, sums.y, cf_w);
+              st_closed += (unsigned)cnt;
+              cls = PB_OUT;
+            }
+          }
+        }
+        const unsigned rm = __ballot_sync(0xffffffffu, cls != PB_OUT);
+        if (cls != PB_OUT)
+          out[nrec + __popc(rm & ((1u << lane) - 1u))] =
+              make_int4(ch | (cls << 8) | (kind << 10), fastw,
+                        pb_pack_win(win[0]) | (pb_pack_win(win[1]) << 16), pb_pack_win(win[2]) | (pb_pack_win(win[3]) << 16));
+        nrec += __popc(rm);
+      }
+      cf_spill();   // bounds the per-lane 32-bit count
+      cf_bin = -1;
+    } else if (stop) {   // (not reached: q_end <= this rank's item count) pass B must still see an empty item
+      if (lane == 0) P.rec_cnt[q - P.q_begin] = 0;
+      break;
+    }
+    if (lane == 0) P.rec_cnt[q - P.q_begin] = nrec;
+  }
+  flush_hist(cur_cat);
+  if (st_closed) atomicAdd(&g_pb_stats[0], 32ull * st_closed);
 }
 
 // Pre-pass: bounding box and sums of every 32-point chunk of every catalogue (one warp per chunk).
@@ -1383,8 +1602,30 @@ pairbin_boxes_kernel(const double* __restrict__ px, const double* __restrict__ p
 
 extern "C" int tgp_pairbin_tile(void) { return PB_CHUNK; }
 
+// Records of one round of the two-pass TwoD count (16 bytes each): 2^26 = 1 GiB, about 8 rounds at N = 1e6.
+constexpr int64_t PB_REC_CAP = 1ll << 26;
+static int64_t g_pb_rec_cap = PB_REC_CAP;   // tgp_set_option("pairbin_record_cap", n): smaller rounds (tests)
+extern "C" int tgp_pairbin_set_record_cap(int n) {
+  g_pb_rec_cap = n <= 0 ? PB_REC_CAP : (n < 256 ? 256 : n);
+  return TGP_OK;
+}
+
+// Record slots reserved in the work buffer for catalogues of up to `max_len` points: an item holds at most `run`
+// records, and run x (items of one catalogue) <= (nblk + 512)^2 / 2 for run <= 256; capped at PB_REC_CAP.
+// Non-decreasing in max_len, so the total point count of the caller's sizing bounds max_cat_len's.
+static int64_t pb_rec_slots(int64_t max_len, int32_t ncat) {
+  const double nblk = (double)((max_len + PB_CHUNK - 1) / PB_CHUNK);
+  const double need = 0.5 * (double)ncat * (nblk + 512.0) * (nblk + 512.0);
+  if (need >= (double)PB_REC_CAP) return PB_REC_CAP;
+  return ((int64_t)need + 255) / 256 * 256;
+}
+// Work buffer of the two-pass count: {2 work counters, 2 spare words} {record counts of a round: slots / 32 ints}
+// {records: 2 doubles each} {pre-pass chunk records}.  The other paths keep the chunk records at the start.
+static int64_t pb_rec_region_doubles(int64_t slots) { return 4 + slots / 64 + 2 * slots; }
+
 extern "C" int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat) {
-  return (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2);
+  return pb_rec_region_doubles(pb_rec_slots(total_points, ncat)) +
+         (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2);
 }
 
 static int g_pb_fast_paths = 7;   // tgp_set_option("pairbin_fast_paths", bits): see PBParams::fast_paths
@@ -1479,16 +1720,74 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
   int64_t grid = tgp_cdiv(P.my_items, warps);
   if (grid > grid_target) grid = grid_target;
 
+  // TwoD block forms need the pre-pass: two passes per round of items, records and counters in `work`
+  const bool split = twod && P.block_sums && work;
+  const int64_t rec_slots = split ? pb_rec_slots(max_cat_len, ncat) : 0;
   P.boxes = nullptr;
   P.sorted = nullptr;
+  P.q_begin = 0;
+  P.q_end = P.my_items;
+  P.recs = nullptr;
+  P.rec_cnt = nullptr;
+  P.counter_next = nullptr;
   if (work) {
     TGP_CHECK_ARG(((uintptr_t)work % 32) == 0, "work must be 32-byte aligned");
+    double* bx = work + (split ? pb_rec_region_doubles(rec_slots) : 0);
     const int64_t warps_needed = nblk * ncat;
     pairbin_boxes_kernel<<<(unsigned)tgp_cdiv(warps_needed * 32, 256), 256, 0, st>>>(px, py, pk, pw, cat_off, ncat, nblk,
-                                                                                       work, work + PB_SLOT);
+                                                                                       bx, bx + PB_SLOT);
     TGP_LAUNCH_CHECK();
-    P.boxes = work;
-    P.sorted = work + PB_SLOT;
+    P.boxes = bx;
+    P.sorted = bx + PB_SLOT;
+  }
+
+  if (split) {
+    // [0] pass A's work counter, [1] pass B's
+    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(work);
+    P.rec_cnt = reinterpret_cast<int*>(work + 4);
+    P.recs = reinterpret_cast<int4*>(work + 4 + rec_slots / 64);
+    const int64_t per_round = (rec_slots < g_pb_rec_cap ? rec_slots : g_pb_rec_cap) / run;   // items
+    TGP_CUDA(cudaMemsetAsync(ctr, 0, 2 * sizeof(unsigned long long), st));
+    PBParams PA = P;
+    // pass A: warp histograms only (forward entries; bins x (count + sum [+ sum w])), as many warps per CTA as the
+    // budget allows (up to 8): every nbins the residual kernel accepts runs
+    const size_t per_warp_a = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0));
+    int warps_a = (int)((budget - fixed - 64) / per_warp_a);
+    if (warps_a > PB_MAX_WARPS) warps_a = PB_MAX_WARPS;
+    PA.warps = warps_a;
+    PA.counter = ctr;
+    PA.counter_next = ctr + 1;
+    const size_t smem_a = fixed + (size_t)warps_a * per_warp_a + 64;   // warps_a >= 1: per_warp_a < the checked per_warp
+    int ctas_a = (int)((220 * 1024) / smem_a);
+    if (ctas_a > PB_CLASSIFY_MIN_CTAS) ctas_a = PB_CLASSIFY_MIN_CTAS;
+    if (ctas_a < 1) ctas_a = 1;
+    P.counter = ctr + 1;
+    P.counter_next = ctr;
+    static TgpPerDeviceOnce once_[2];
+    const void* kern_a = weighted ? (const void*)pairbin_classify_kernel<true> : (const void*)pairbin_classify_kernel<false>;
+    const void* kern_b = weighted ? (const void*)pairbin_kernel<TGP_BIN_TWOD, true, true>
+                                  : (const void*)pairbin_kernel<TGP_BIN_TWOD, false, true>;
+    if (tgp_first_use_on_device(once_[weighted ? 1 : 0])) {
+      TGP_CUDA(cudaFuncSetAttribute(kern_a, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
+      TGP_CUDA(cudaFuncSetAttribute(kern_b, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
+    }
+    for (int64_t q0 = 0; q0 < P.my_items; q0 += per_round) {
+      const int64_t q1 = (q0 + per_round < P.my_items) ? q0 + per_round : P.my_items;
+      PA.q_begin = P.q_begin = q0;
+      PA.q_end = P.q_end = q1;
+      int64_t grid_a = tgp_cdiv(q1 - q0, warps_a), grid_b = tgp_cdiv(q1 - q0, warps);
+      if (grid_a > (int64_t)sms * ctas_a) grid_a = (int64_t)sms * ctas_a;
+      if (grid_b > grid_target) grid_b = grid_target;
+      if (weighted) {
+        pairbin_classify_kernel<true><<<(unsigned)grid_a, warps_a * 32, smem_a, st>>>(PA);
+        pairbin_kernel<TGP_BIN_TWOD, true, true><<<(unsigned)grid_b, warps * 32, smem, st>>>(P);
+      } else {
+        pairbin_classify_kernel<false><<<(unsigned)grid_a, warps_a * 32, smem_a, st>>>(PA);
+        pairbin_kernel<TGP_BIN_TWOD, false, true><<<(unsigned)grid_b, warps * 32, smem, st>>>(P);
+      }
+      TGP_LAUNCH_CHECK();
+    }
+    return TGP_OK;
   }
 
   static std::atomic<unsigned> launch_seq{0};   // host threads launching on different streams get different slots
@@ -1506,9 +1805,7 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
                                     (int)budget));                                                        \
     pairbin_kernel<BT, W, BS><<<(unsigned)grid, warps * 32, smem, st>>>(P);                               \
   } while (0)
-  if (twod && P.block_sums) {
-    if (weighted) TGP_PB_LAUNCH(TGP_BIN_TWOD, true, true); else TGP_PB_LAUNCH(TGP_BIN_TWOD, false, true);
-  } else if (twod) {
+  if (twod) {   // pair by pair (block forms off, or no work buffer for the pre-pass)
     if (weighted) TGP_PB_LAUNCH(TGP_BIN_TWOD, true, false); else TGP_PB_LAUNCH(TGP_BIN_TWOD, false, false);
   } else {
     if (P.block_sums) {
