@@ -310,8 +310,9 @@ typedef enum {
  *                   pre-pass; for TwoD also the block records and work counters of the two-pass count, see
  *                   below).  NULL: no block forms (TwoD: pair by pair; Log: the boxes are recomputed on the fly);
  *                   the counts are the same.
- * TwoD with work runs in rounds of this rank's items: a classification pass books the blocks that sit in one
- * bin and records the others, then a second kernel processes the recorded blocks.  A round holds at most
+ * TwoD with work first books the pairs of super-chunks (256 consecutive points) that sit in one bin or vary along
+ * one axis only, then runs in rounds of this rank's items: a classification pass books the other blocks that sit
+ * in one bin and records the rest, then a second kernel processes the recorded blocks.  A round holds at most
  * 2^26 records (1 GiB of `work` at N >= ~4e5; fewer for smaller catalogues), about 8 rounds at N = 1e6. */
 int tgp_pairbin(const double* px, const double* py, const double* pk, const double* pw,
                 const int64_t* cat_off, int32_t ncat, int64_t max_cat_len, int32_t bin_type,
@@ -320,7 +321,8 @@ int tgp_pairbin(const double* px, const double* py, const double* pk, const doub
                 double* sumwkk, double* sumwr, double* work, void* stream);
 
 /* Size (in doubles) of the optional scratch buffer of tgp_pairbin for catalogues of `total_points` points in
- * all (an upper bound on max_cat_len is enough): the chunk records of the pre-pass plus the block records of one
+ * all (an upper bound on max_cat_len is enough): the chunk records of the pre-pass, the super-chunk records
+ * (boxes, sums and sorted copies of 256-point super-chunks, about 48 MB at N = 1e6) and the block records of one
  * round, capped at 2^26 records of 16 bytes. */
 int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat);
 
@@ -438,7 +440,9 @@ int tgp_pairbin_tile(void);
  * varying axis (one compare pair per pair of points), [2] pair by pair in a 2 x 2 bin window or through the
  * generic path (the diagonal blocks are not tallied), [3] one varying axis answered by a rank query on the
  * chunk's sorted copy (8 probes per row point instead of 32 compares), [4] 2 x 2 bin window with the column-bit
- * and row-bit sums from two such rank queries and only the "both bits" quadrant summed pair by pair.  Synchronous. */
+ * and row-bit sums from two such rank queries and only the "both bits" quadrant summed pair by pair, [5] (TwoD)
+ * super-chunk pair in one bin, booked whole, [6] (TwoD) super-chunk pair with one varying axis, one rank query per row
+ * point on the super-chunk's sorted copy.  The slots are disjoint.  Synchronous. */
 int tgp_pairbin_stats(unsigned long long* host8 /*host*/, int reset);
 
 /* Tuning knobs for experiments (not needed for normal use).  "trsv_cluster": thread-block cluster size of the

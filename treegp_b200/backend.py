@@ -779,7 +779,8 @@ def pairbin_stats(reset=True):
     """Pairs per kernel path since the last reset (see tgp_pairbin_stats); synchronises the device."""
     buf = (ctypes.c_ulonglong * 8)()
     check(_cabi.load().tgp_pairbin_stats(buf, int(bool(reset))), "tgp_pairbin_stats")
-    keys = ("closed_form", "one_axis", "pairwise", "one_axis_sorted", "two_axis_sorted")
+    keys = ("closed_form", "one_axis", "pairwise", "one_axis_sorted", "two_axis_sorted", "super_closed_form",
+            "super_one_axis")
     return {k: int(buf[i]) for i, k in enumerate(keys)}
 
 

@@ -26,6 +26,9 @@
 // block from the chunk boxes, books the closed-form blocks and records the others; pairbin_kernel<TwoD, W, true> then
 // runs the paths below over the recorded blocks only.  The classification needs none of the per-row register state
 // of the residual paths, so it runs at more warps per SM and the residual kernel's warm code no longer contains it.
+// Before the rounds, pairbin_super_kernel books the pairs of super-chunks (PB_SUPER chunks) that are out of range, sit
+// in one bin, or vary along one axis only (one rank query per row point on the super-chunk's sorted copy); the
+// classification pass skips their blocks and descends to the 32-point blocks only for the other super pairs.
 //
 // Two instantiations per bin type (template parameter BS):
 //   BS = false  the pair-by-pair kernel: every pair of every in-range block is evaluated individually
@@ -68,6 +71,16 @@ constexpr int PB_FLUSH_ITEMS = 2048;  // keeps the 32-bit private counters from 
 constexpr int PB_SLOT = 8;            // doubles per chunk slot of the pre-pass: box + sums
 constexpr int PB_SORTED = 6 * PB_CHUNK;  // + {sorted x, suffix k w, suffix w, sorted y, suffix k w, suffix w}
 constexpr int PB_STRIDE = PB_SLOT + PB_SORTED;   // the two records of a chunk are stored back to back
+// Super-chunks (TwoD block forms): PB_SUPER consecutive chunks of a catalogue, aligned to chunk 0.  Only full ones
+// (PB_SUPER_PTS points) get a record: {box, sum k w, sum w, -, -} + the points sorted by x and by y, each with suffix
+// sums of k w and w.  8 was the fastest admissible size at the bench size (DESIGN section 5, v10).
+#ifndef PB_SUPER
+#define PB_SUPER 8
+#endif
+constexpr int PB_SUPER_PTS = PB_SUPER * PB_CHUNK;
+constexpr int PB_SUPER_STRIDE = PB_SLOT + 6 * PB_SUPER_PTS;
+// the warp histogram of the super kernel takes <= 32 x PB_SUPER_PTS^2 pairs per item: flush before 2^31
+constexpr int PB_SUPER_FLUSH_ITEMS = (int)((1u << 31) / (32u * PB_SUPER_PTS * PB_SUPER_PTS));
 
 struct PBParams {
   const double *px, *py, *pk, *pw;
@@ -85,7 +98,8 @@ struct PBParams {
   int64_t my_items;       // number of work items of this rank
   int32_t run;            // column chunks per work item (multiple of 32)
   int32_t ncat, nbins, nb, warps, rank, nranks;
-  int32_t block_sums;     // 1: blocks whose pairs provably share a window bit use the block forms (default)
+  int32_t block_sums;     // 1: blocks whose pairs provably share a window bit use the block forms (default); 2 (TwoD
+                          // classification pass only): and the super pairs that are not DESCEND go to the super kernel
   int32_t fast_paths;     // bit 0: short-cut dispatch of one-axis blocks that fit the open window; bit 1: 2 x 2-window
                           // blocks with marginal sums from rank queries; bit 2: pair-by-pair kernel, no mirrored bits
                           // per pair in blocks that provably sit in one bin and its mirror image (default: all)
@@ -102,7 +116,8 @@ struct PBParams {
 // tallied by the classification pass, the others by the pass over the recorded blocks),
 // [1] one varying axis, pair by pair, [2] pair by pair (2 x 2 window with or without the per-pair range test,
 // generic sub-blocks), [3] one varying axis answered by a rank query on the sorted chunk, [4] 2 x 2 window with the
-// marginal sums from rank queries (one quadrant pair by pair).  Diagnostics.
+// marginal sums from rank queries (one quadrant pair by pair), [5] super pair in one bin, [6] super pair with one
+// varying axis (rank queries on the super-chunk's sorted copy).  Diagnostics.
 __device__ unsigned long long g_pb_stats[8];
 
 __device__ __forceinline__ int pb_bin_twod(double d, double hi, double inv_bin, int nbins,
@@ -1393,6 +1408,44 @@ pairbin_kernel(PBParams P) {
 #ifndef PB_CLASSIFY_MIN_CTAS
 #define PB_CLASSIFY_MIN_CTAS 2
 #endif
+
+// The super records follow the chunk records; their start depends on the total point count cat_off[ncat].
+__device__ __forceinline__ const double* pb_super_records(const PBParams& P) {
+  return P.boxes + (size_t)PB_STRIDE * (size_t)(P.cat_off[P.ncat] / PB_CHUNK + P.ncat + 2);
+}
+
+// Status of super pair (R, C) of one catalogue from the super boxes (srec = record of super-chunk 0 of the catalogue,
+// nsf = its number of full super-chunks).  Exact for the reason the chunk classification is: FP subtraction is
+// monotone, so the boxes bound every displacement.
+//   OUT       every pair fails the range test;
+//   CLOSED    every pair in range, in ONE forward bin per axis, and the mirrored window is its mirror image;
+//   ONE_AXIS  every pair in range, one such bin on one axis, exactly two forward bins [v0, v0 + 1] on the other whose
+//             mirrored window is the mirror image [nbins-2-v0, nbins-1-v0]; vx: x is the varying axis;
+//   DESCEND   anything else, the diagonal (R == C) and short super-chunks: the chunks are classified one by one.
+// The super kernel books the first three; the classification pass skips every block of such a pair.
+enum { PB_S_OUT = 0, PB_S_CLOSED = 1, PB_S_ONE_AXIS = 2, PB_S_DESCEND = 3 };
+__device__ __forceinline__ int pb_super_status(const double* __restrict__ srec, int64_t nsf, int64_t R, int64_t C,
+                                               double M, double lo2, int nbins, const double* __restrict__ ed,
+                                               int& x0, int& y0, bool& vx) {
+  if (R == C || R >= nsf || C >= nsf) return PB_S_DESCEND;
+  const double4 a = *reinterpret_cast<const double4*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)R);
+  const double4 b = *reinterpret_cast<const double4*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)C);
+  int w[4];
+  const int cls = pb_classify_twod<true>(a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, M, lo2, nbins, ed, w);
+  if (cls == PB_OUT) return PB_S_OUT;
+  if (cls != PB_REG_FULL) return PB_S_DESCEND;
+  x0 = w[0] & 0xffff;
+  y0 = w[1] & 0xffff;
+  const int rx0 = w[2] & 0xffff, ry0 = w[3] & 0xffff;
+  const bool one_x = (w[0] >> 16) == 0 && (w[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
+  const bool one_y = (w[1] >> 16) == 0 && (w[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
+  const bool clean_x = (w[0] >> 16) == 1 && (w[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
+  const bool clean_y = (w[1] >> 16) == 1 && (w[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
+  vx = one_y;
+  if (one_x && one_y) return PB_S_CLOSED;
+  if ((one_y && clean_x) || (one_x && clean_y)) return PB_S_ONE_AXIS;
+  return PB_S_DESCEND;
+}
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_CLASSIFY_MIN_CTAS)
 pairbin_classify_kernel(PBParams P) {
@@ -1483,52 +1536,74 @@ pairbin_classify_kernel(PBParams P) {
       const double2 rsum = *reinterpret_cast<const double2*>(rec0 + (size_t)PB_STRIDE * (size_t)it.ib + 4);
       const int nlive = (it.ib == nblk - 1) ? tail : PB_CHUNK;
       int4* out = P.recs + (size_t)(q - P.q_begin) * (size_t)P.run;
-      for (int s0 = 0; s0 < span; s0 += 32) {
-        const int ch = s0 + lane;   // chunk c_lo + ch
-        int cls = PB_OUT, kind = 0, fastw = 0;
-        int win[4] = {0, 0, 0, 0};
-        if (ch < span) {
-          const double* rec = recl + (size_t)PB_STRIDE * (size_t)ch;
-          const int cnt = (ch == last) ? tail : PB_CHUNK;
-          const double4 bb = *reinterpret_cast<const double4*>(rec);
-          if (diag && ch == 0) cls = PB_GENERIC;  // diagonal block: needs j > i
-          else cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, bb.x, bb.y, bb.z, bb.w, M, lo2, nbins, ed, win);
-          if (cls == PB_REG_FULL) {
-            const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
-            const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
-            const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
-            // exactly one varying axis: the block is answered from the chunk's points sorted along that axis
-            if (cnt == PB_CHUNK) kind = (one_y && !one_x) ? 1 : ((one_x && !one_y) ? 2 : 0);
-            // kind != 0 and the varying axis spans exactly two forward bins [v0, v0+1] whose mirrored window is the
-            // mirror image (the usual case): 1 | kind << 1 | x0 << 3 | y0 << 15, everything pass B needs to see
-            // whether its open window covers the block
-            if (P.fast_paths & 1) {
-              const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
-              const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
-              if ((kind == 1 && clean_x) || (kind == 2 && clean_y)) fastw = 1 | (kind << 1) | (x0 << 3) | (y0 << 15);
-            }
-            // two bins along BOTH axes: the raw points are staged (kind stays 0); field value 3
-            if ((P.fast_paths & 2) && cnt == PB_CHUNK && (win[0] >> 16) == 1 && (win[2] >> 16) == 1 &&
-                rx0 == nbins - 2 - x0 && (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0)
-              fastw = 1 | (3 << 1) | (x0 << 3) | (y0 << 15);
-            if (one_x && one_y) {
-              const double2 sums = *reinterpret_cast<const double2*>(rec + 4);
-              const int o = y0 * nbins + x0;
-              if (o != cf_bin) { cf_spill(); cf_bin = o; }
-              cf_cnt += (unsigned)(nlive * cnt);
-              cf_s = fma(rsum.x, sums.x, cf_s);
-              if constexpr (WEIGHTED) cf_w = fma(rsum.y, sums.y, cf_w);
-              st_closed += (unsigned)cnt;
-              cls = PB_OUT;
+      // the super kernel books every super pair that is not DESCEND (on one rank); its blocks are skipped here on every
+      // rank.  Lane l decides super column cw + l; the chunks of the DESCEND ones are then classified 32 at a time.
+      const double* srec = pb_super_records(P) + (size_t)PB_SUPER_STRIDE * (size_t)(it.off / PB_SUPER_PTS + it.cat);
+      const int64_t nsf = P.block_sums == 2 ? it.n / PB_SUPER_PTS : 0, sR = it.ib / PB_SUPER;
+      for (int64_t cw = it.c_lo / PB_SUPER; cw * PB_SUPER < it.c_hi; cw += 32) {
+        int sx0, sy0;
+        bool svx;
+        const unsigned dm = __ballot_sync(0xffffffffu, (cw + lane) * PB_SUPER < it.c_hi &&
+            pb_super_status(srec, nsf, sR, cw + lane, M, lo2, nbins, ed, sx0, sy0, svx) == PB_S_DESCEND);
+        const int nd = __popc(dm) * PB_SUPER;
+        const int base = (int)(cw * PB_SUPER - it.c_lo);   // negative only for the diagonal super-chunk
+        for (int s0 = 0; s0 < nd; s0 += 32) {
+          int ch = span;   // chunk c_lo + ch: the ((s0 + lane) % PB_SUPER)-th chunk of the ((s0 + lane) / PB_SUPER)-th
+          if (s0 + lane < nd) {   // DESCEND super column: bit b of dm is its t-th set bit <=> popc(dm below b) == t
+            const int t = (s0 + lane) / PB_SUPER;
+            int b = 0;
+#pragma unroll
+            for (int step = 16; step > 0; step >>= 1)
+              if (__popc(dm & ((1u << (b + step)) - 1u)) <= t) b += step;
+            const int c = base + b * PB_SUPER + (s0 + lane) % PB_SUPER;
+            if (c >= 0 && c < span) ch = c;
+          }
+          int cls = PB_OUT, kind = 0, fastw = 0;
+          int win[4] = {0, 0, 0, 0};
+          if (ch < span) {
+            const double* rec = recl + (size_t)PB_STRIDE * (size_t)ch;
+            const int cnt = (ch == last) ? tail : PB_CHUNK;
+            const double4 bb = *reinterpret_cast<const double4*>(rec);
+            if (diag && ch == 0) cls = PB_GENERIC;  // diagonal block: needs j > i
+            else cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, bb.x, bb.y, bb.z, bb.w, M, lo2, nbins, ed, win);
+            if (cls == PB_REG_FULL) {
+              const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
+              const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
+              const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
+              // exactly one varying axis: the block is answered from the chunk's points sorted along that axis
+              if (cnt == PB_CHUNK) kind = (one_y && !one_x) ? 1 : ((one_x && !one_y) ? 2 : 0);
+              // kind != 0 and the varying axis spans exactly two forward bins [v0, v0+1] whose mirrored window is the
+              // mirror image (the usual case): 1 | kind << 1 | x0 << 3 | y0 << 15, everything pass B needs to see
+              // whether its open window covers the block
+              if (P.fast_paths & 1) {
+                const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
+                const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
+                if ((kind == 1 && clean_x) || (kind == 2 && clean_y)) fastw = 1 | (kind << 1) | (x0 << 3) | (y0 << 15);
+              }
+              // two bins along BOTH axes: the raw points are staged (kind stays 0); field value 3
+              if ((P.fast_paths & 2) && cnt == PB_CHUNK && (win[0] >> 16) == 1 && (win[2] >> 16) == 1 &&
+                  rx0 == nbins - 2 - x0 && (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0)
+                fastw = 1 | (3 << 1) | (x0 << 3) | (y0 << 15);
+              if (one_x && one_y) {
+                const double2 sums = *reinterpret_cast<const double2*>(rec + 4);
+                const int o = y0 * nbins + x0;
+                if (o != cf_bin) { cf_spill(); cf_bin = o; }
+                cf_cnt += (unsigned)(nlive * cnt);
+                cf_s = fma(rsum.x, sums.x, cf_s);
+                if constexpr (WEIGHTED) cf_w = fma(rsum.y, sums.y, cf_w);
+                st_closed += (unsigned)cnt;
+                cls = PB_OUT;
+              }
             }
           }
+          const unsigned rm = __ballot_sync(0xffffffffu, cls != PB_OUT);
+          if (cls != PB_OUT)
+            out[nrec + __popc(rm & ((1u << lane) - 1u))] =
+                make_int4(ch | (cls << 8) | (kind << 10), fastw,
+                          pb_pack_win(win[0]) | (pb_pack_win(win[1]) << 16),
+                          pb_pack_win(win[2]) | (pb_pack_win(win[3]) << 16));
+          nrec += __popc(rm);
         }
-        const unsigned rm = __ballot_sync(0xffffffffu, cls != PB_OUT);
-        if (cls != PB_OUT)
-          out[nrec + __popc(rm & ((1u << lane) - 1u))] =
-              make_int4(ch | (cls << 8) | (kind << 10), fastw,
-                        pb_pack_win(win[0]) | (pb_pack_win(win[1]) << 16), pb_pack_win(win[2]) | (pb_pack_win(win[3]) << 16));
-        nrec += __popc(rm);
       }
       cf_spill();   // bounds the per-lane 32-bit count
       cf_bin = -1;
@@ -1600,6 +1675,258 @@ pairbin_boxes_kernel(const double* __restrict__ px, const double* __restrict__ p
   }
 }
 
+// Pre-pass of the super-chunks: one CTA of PB_SUPER_PTS threads per full super-chunk sorts its points by x and by y
+// (bitonic network in shared memory) and stores them with the suffix sums of k w and w, the box (the sorted ends) and
+// the sums (the first suffix sums of the x order).  Record of super-chunk s of catalogue `cat`:
+// PB_SUPER_STRIDE x (cat_off[cat] / PB_SUPER_PTS + s + cat) doubles from the start of the super records, which
+// follow the chunk records (`boxes`).
+__global__ void __launch_bounds__(PB_SUPER_PTS)
+pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restrict__ py, const double* __restrict__ pk,
+                           const double* __restrict__ pw, const int64_t* __restrict__ cat_off, int32_t ncat,
+                           int64_t supers_per_cat, double* __restrict__ boxes) {
+  __shared__ double s_key[PB_SUPER_PTS], s_k[PB_SUPER_PTS], s_w[PB_SUPER_PTS], s_part[2][PB_SUPER_PTS / 32];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const int64_t cat = blockIdx.x / supers_per_cat, s = blockIdx.x % supers_per_cat;
+  if (cat >= ncat) return;
+  const int64_t off = cat_off[cat], n = cat_off[cat + 1] - off;
+  if ((s + 1) * PB_SUPER_PTS > n) return;   // only full super-chunks take a super form
+  const int64_t j = off + s * PB_SUPER_PTS + t;
+  const double wj = pw ? pw[j] : 1.0, kj = pk[j] * wj;
+  double* o = boxes + (size_t)PB_STRIDE * (size_t)(cat_off[ncat] / PB_CHUNK + ncat + 2) +   // = pb_super_records
+              (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + s + cat);
+  for (int axis = 0; axis < 2; ++axis) {
+    s_key[t] = axis == 0 ? px[j] : py[j];
+    s_k[t] = kj;
+    s_w[t] = wj;
+    __syncthreads();
+    for (int k2 = 2; k2 <= PB_SUPER_PTS; k2 <<= 1) {
+      for (int j2 = k2 >> 1; j2 > 0; j2 >>= 1) {
+        const int u = t ^ j2;
+        if (u > t) {
+          const bool up = (t & k2) == 0;
+          if (up ? (s_key[t] > s_key[u]) : (s_key[t] < s_key[u])) {
+            double v = s_key[t]; s_key[t] = s_key[u]; s_key[u] = v;
+            v = s_k[t]; s_k[t] = s_k[u]; s_k[u] = v;
+            v = s_w[t]; s_w[t] = s_w[u]; s_w[u] = v;
+          }
+        }
+        __syncthreads();
+      }
+    }
+    // suffix sums: within the warp, then the totals of the warps above
+    double vk = s_k[t], vw = s_w[t];
+#pragma unroll
+    for (int o2 = 1; o2 < 32; o2 <<= 1) {
+      const double tk = __shfl_down_sync(0xffffffffu, vk, o2), tw = __shfl_down_sync(0xffffffffu, vw, o2);
+      if (lane + o2 < 32) { vk += tk; vw += tw; }
+    }
+    if (lane == 0) { s_part[0][warp] = vk; s_part[1][warp] = vw; }
+    __syncthreads();
+    for (int u = warp + 1; u < PB_SUPER_PTS / 32; ++u) { vk += s_part[0][u]; vw += s_part[1][u]; }
+    double* so = o + PB_SLOT + axis * 3 * PB_SUPER_PTS + t;
+    so[0] = s_key[t];
+    so[PB_SUPER_PTS] = vk;
+    so[2 * PB_SUPER_PTS] = vw;
+    if (t == 0) {
+      o[2 * axis] = s_key[0];
+      o[2 * axis + 1] = s_key[PB_SUPER_PTS - 1];
+      if (axis == 0) { o[4] = vk; o[5] = vw; o[6] = 0.0; o[7] = 0.0; }
+    }
+    __syncthreads();   // the buffers are refilled for the y order
+  }
+}
+
+// The super kernel: books every super pair that is not DESCEND, once per count, before the rounds.  Items are (super
+// row R, run of 32 super columns) of this rank, dealt like the chunk items; lane l takes the status of super pair
+// (R, 32 r + l).
+//   CLOSED    booked by its lane: count n_R n_C, sum (sum k w)_R (sum k w)_C (forward entry only);
+//   ONE_AXIS  one pair at a time by the warp: the column super-chunk's copy sorted along the varying axis is staged in
+//             shared memory, and every row point i finds pos = #{j : fl(c_j - c_i) < t} by bisection with that
+//             predicate (monotone in c_j).  The upper bin gets n_C - pos pairs and k_i w_i x suffix(pos), the lower bin
+//             the rest.  The exact mirrored bits differ from the mirror image only for the columns between pos and
+//             pos_m = #{j : fl(c_j - c_i) <= -t_m}, nearly always none; those pairs are moved in global memory.
+// The warp histograms hold forward entries; the mirror image is added when they are written out.
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(PB_MAX_WARPS * 32, 2)
+pairbin_super_kernel(PBParams P) {
+  extern __shared__ __align__(16) unsigned char pb_smem[];
+  const int nb = P.nb, nbins = P.nbins;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  double* ed = reinterpret_cast<double*>(pb_smem);                        // nbins + 1 (padded to even)
+  double* stage_all = ed + ((nbins + 2) & ~1);                            // [warps][3][PB_SUPER_PTS]
+  double* hs_all = stage_all + (size_t)P.warps * 3 * PB_SUPER_PTS;        // [warps][nb]  sum wk wk
+  double* hw_all = hs_all + (size_t)P.warps * nb;                         // [warps][nb]  sum w w     (WEIGHTED)
+  unsigned* hc_all = reinterpret_cast<unsigned*>(hw_all + (WEIGHTED ? (size_t)P.warps * nb : 0));
+  double* sc = stage_all + (size_t)warp * 3 * PB_SUPER_PTS;   // sorted coordinates
+  double* ss = sc + PB_SUPER_PTS;                             // suffix sums of k w
+  double* sw = ss + PB_SUPER_PTS;                             // suffix sums of w
+  double* my_s = hs_all + (size_t)warp * nb;
+  double* my_w = hw_all + (size_t)warp * nb;
+  unsigned* my_c = hc_all + (size_t)warp * nb;
+  for (int i = tid; i <= nbins; i += blockDim.x) ed[i] = P.edges[i];
+  for (int i = lane; i < nb; i += 32) {
+    my_s[i] = 0.0;
+    my_c[i] = 0u;
+    if constexpr (WEIGHTED) my_w[i] = 0.0;
+  }
+  __syncthreads();
+
+  auto flush_hist = [&](int cat) {   // forward entries of bin b + those of its mirror image, then clear
+    __syncwarp();
+    if (cat >= 0) {
+      for (int b = lane; b < nb; b += 32) {
+        const int bm = nb - 1 - b;
+        const unsigned long long c = (unsigned long long)my_c[b] + (unsigned long long)my_c[bm];
+        if (c) {
+          const size_t o = (size_t)cat * nb + b;
+          atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + o, c);
+          atomicAdd(P.sumwkk + o, my_s[b] + my_s[bm]);
+          atomicAdd(P.sumw + o, WEIGHTED ? my_w[b] + my_w[bm] : (double)c);
+        }
+      }
+      __syncwarp();
+      for (int b = lane; b < nb; b += 32) {
+        my_c[b] = 0u;
+        my_s[b] = 0.0;
+        if constexpr (WEIGHTED) my_w[b] = 0.0;
+      }
+    }
+    __syncwarp();
+  };
+
+  const double M = P.hi, lo2 = P.lo2;
+  const double* sup0 = pb_super_records(P);
+  const int64_t nruns = (P.items_per_cat + 31) / 32;   // items_per_cat: super-chunks of the longest catalogue
+  unsigned st_closed = 0, st_one = 0;   // super pairs
+  int cur_cat = -1, since_flush = 0;
+  while (true) {
+    unsigned long long q = 0;
+    if (lane == 0) q = atomicAdd(P.counter, 1ull);
+    q = __shfl_sync(0xffffffffu, q, 0);
+    if ((int64_t)q >= P.my_items) break;
+    const int64_t item = (int64_t)q * P.nranks + P.rank;
+    const int cat = (int)(item / (P.items_per_cat * nruns));
+    if (cat >= P.ncat) break;
+    const int64_t R = (item % (P.items_per_cat * nruns)) / nruns, r = item % nruns;
+    const int64_t off = P.cat_off[cat], n = P.cat_off[cat + 1] - off;
+    const int64_t nsf = n / PB_SUPER_PTS;
+    if (R >= nsf || (r + 1) * 32 <= R + 1 || r * 32 >= nsf) continue;   // no super column C > R in this run
+    if (cat != cur_cat || since_flush >= PB_SUPER_FLUSH_ITEMS) {
+      flush_hist(cur_cat);
+      cur_cat = cat;
+      since_flush = 0;
+    }
+    ++since_flush;
+    const double* srec = sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat);
+    const double* rrec = srec + (size_t)PB_SUPER_STRIDE * (size_t)R;
+    const double2 rsum = *reinterpret_cast<const double2*>(rrec + 4);
+    const int64_t C = r * 32 + lane;
+    int x0 = 0, y0 = 0;
+    bool vx = false;
+    const int st = C > R ? pb_super_status(srec, nsf, R, C, M, lo2, nbins, ed, x0, y0, vx) : PB_S_DESCEND;
+    if (st == PB_S_CLOSED) {
+      const double2 csum = *reinterpret_cast<const double2*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)C + 4);
+      const int o = y0 * nbins + x0;
+      atomicAdd(my_c + o, (unsigned)(PB_SUPER_PTS * PB_SUPER_PTS));
+      atomicAdd(my_s + o, rsum.x * csum.x);
+      if constexpr (WEIGHTED) atomicAdd(my_w + o, rsum.y * csum.y);
+      ++st_closed;
+    }
+    unsigned todo = __ballot_sync(0xffffffffu, st == PB_S_ONE_AXIS);
+    while (todo) {
+      const int c = __ffs(todo) - 1;
+      todo &= todo - 1;
+      const bool cvx = __shfl_sync(0xffffffffu, vx, c);
+      const int cx0 = __shfl_sync(0xffffffffu, x0, c), cy0 = __shfl_sync(0xffffffffu, y0, c);
+      const double* crec = srec + (size_t)PB_SUPER_STRIDE * (size_t)(r * 32 + c);
+      const double* srt = crec + PB_SLOT + (cvx ? 0 : 3 * PB_SUPER_PTS);
+      __syncwarp();   // the previous pair's staging is consumed
+      for (int u = lane; u < PB_SUPER_PTS; u += 32) {
+        sc[u] = srt[u];
+        ss[u] = srt[PB_SUPER_PTS + u];
+        if constexpr (WEIGHTED) sw[u] = srt[2 * PB_SUPER_PTS + u];
+      }
+      __syncwarp();
+      const int v0 = cvx ? cx0 : cy0, cb = cvx ? cy0 : cx0;   // varying axis: bins v0, v0 + 1; constant axis: bin cb
+      const double t = ed[v0 + 1], tm = -ed[nbins - 1 - v0];   // forward upper bit: d >= t; mirrored upper bit: d <= tm
+      const double* rc = (cvx ? P.px : P.py) + off + R * PB_SUPER_PTS;
+      const double* rk = P.pk + off + R * PB_SUPER_PTS;
+      const double* rw = WEIGHTED ? P.pw + off + R * PB_SUPER_PTS : nullptr;
+      double up_s = 0.0, up_w = 0.0;
+      unsigned up_c = 0u;
+#pragma unroll 2
+      for (int k = 0; k < PB_SUPER; ++k) {
+        const int i = k * 32 + lane;
+        const double ci = rc[i];
+        double wi = 1.0;
+        if constexpr (WEIGHTED) wi = rw[i];
+        const double ki = rk[i] * wi;
+        // pos = #{j : fl(c_j - c_i) < t} (branch-free lower bound over the ascending copy)
+        int pos = 0;
+#pragma unroll
+        for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
+          if (__dsub_rn(sc[pos + step - 1], ci) < t) pos += step;
+        if (pos == PB_SUPER_PTS - 1 && __dsub_rn(sc[pos], ci) < t) pos = PB_SUPER_PTS;
+        up_c += (unsigned)(PB_SUPER_PTS - pos);
+        const double sk = pos < PB_SUPER_PTS ? ss[pos] : 0.0;
+        up_s = fma(ki, sk, up_s);
+        double swp = 0.0;
+        if constexpr (WEIGHTED) { swp = pos < PB_SUPER_PTS ? sw[pos] : 0.0; up_w = fma(wi, swp, up_w); }
+        // exact mirrored bits: consistent iff pos_m == pos, i.e. column pos - 1 has the mirrored upper bit and column
+        // pos has not
+        const bool ok = (pos == 0 || __dsub_rn(sc[pos - 1], ci) <= tm) &&
+                        (pos == PB_SUPER_PTS || !(__dsub_rn(sc[pos], ci) <= tm));
+        if (!ok) {   // (rare) a column within rounding of a bin edge
+          int pm = 0;
+          for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
+            if (__dsub_rn(sc[pm + step - 1], ci) <= tm) pm += step;
+          if (pm == PB_SUPER_PTS - 1 && __dsub_rn(sc[pm], ci) <= tm) pm = PB_SUPER_PTS;
+          // columns [lo, hi) have a mirrored bin that is not the mirror image of their forward bin: pm > pos, forward
+          // upper bin whose mirrored entry is the upper mirrored bin; pm < pos, forward lower bin, mirrored lower bin
+          const int a = min(pos, pm), b = max(pos, pm);
+          const double kk = ki * ((a < PB_SUPER_PTS ? ss[a] : 0.0) - (b < PB_SUPER_PTS ? ss[b] : 0.0));
+          double ww = (double)(b - a);
+          if constexpr (WEIGHTED) ww = wi * ((a < PB_SUPER_PTS ? sw[a] : 0.0) - (b < PB_SUPER_PTS ? sw[b] : 0.0));
+          const int fv = pm > pos ? v0 + 1 : v0;                   // forward bin on the varying axis
+          const int av = nbins - 1 - fv;                           // assumed mirrored bin: the mirror image
+          const int xv = pm > pos ? nbins - 1 - v0 : nbins - 2 - v0;   // exact mirrored bin
+          const int mc = nbins - 1 - cb;                           // mirrored bin on the constant axis (exact)
+          const int assumed = cvx ? mc * nbins + av : av * nbins + mc;
+          const int exact = cvx ? mc * nbins + xv : xv * nbins + mc;
+          const size_t g = (size_t)cat * nb;
+          unsigned long long* cnt = reinterpret_cast<unsigned long long*>(P.npairs) + g;
+          atomicAdd(cnt + assumed, (unsigned long long)(-(long long)(b - a)));   // -(b - a) (mod 2^64)
+          atomicAdd(cnt + exact, (unsigned long long)(b - a));
+          atomicAdd(P.sumwkk + g + assumed, -kk);
+          atomicAdd(P.sumwkk + g + exact, kk);
+          atomicAdd(P.sumw + g + assumed, -ww);
+          atomicAdd(P.sumw + g + exact, ww);
+        }
+      }
+      up_c = warp_sum_u(up_c);
+      up_s = warp_sum(up_s);
+      if constexpr (WEIGHTED) up_w = warp_sum(up_w);
+      if (lane == 0) {   // the histogram is private to this warp
+        const double2 csum = *reinterpret_cast<const double2*>(crec + 4);
+        const int lo_b = cvx ? cb * nbins + v0 : v0 * nbins + cb;
+        const int hi_b = cvx ? cb * nbins + v0 + 1 : (v0 + 1) * nbins + cb;
+        my_c[lo_b] += (unsigned)(PB_SUPER_PTS * PB_SUPER_PTS) - up_c;
+        my_s[lo_b] += rsum.x * csum.x - up_s;
+        my_c[hi_b] += up_c;
+        my_s[hi_b] += up_s;
+        if constexpr (WEIGHTED) {
+          my_w[lo_b] += rsum.y * csum.y - up_w;
+          my_w[hi_b] += up_w;
+        }
+        ++st_one;
+      }
+    }
+  }
+  flush_hist(cur_cat);
+  if (st_closed) atomicAdd(&g_pb_stats[5], (unsigned long long)PB_SUPER_PTS * PB_SUPER_PTS * st_closed);
+  if (st_one) atomicAdd(&g_pb_stats[6], (unsigned long long)PB_SUPER_PTS * PB_SUPER_PTS * st_one);
+}
+
 extern "C" int tgp_pairbin_tile(void) { return PB_CHUNK; }
 
 // Records of one round of the two-pass TwoD count (16 bytes each): 2^26 = 1 GiB, about 8 rounds at N = 1e6.
@@ -1619,13 +1946,15 @@ static int64_t pb_rec_slots(int64_t max_len, int32_t ncat) {
   if (need >= (double)PB_REC_CAP) return PB_REC_CAP;
   return ((int64_t)need + 255) / 256 * 256;
 }
-// Work buffer of the two-pass count: {2 work counters, 2 spare words} {record counts of a round: slots / 32 ints}
-// {records: 2 doubles each} {pre-pass chunk records}.  The other paths keep the chunk records at the start.
+// Work buffer of the two-pass count: {3 work counters, 1 spare word} {record counts of a round: slots / 32 ints}
+// {records: 2 doubles each} {pre-pass chunk records} {super-chunk records}.  The other paths keep the chunk records
+// at the start.
 static int64_t pb_rec_region_doubles(int64_t slots) { return 4 + slots / 64 + 2 * slots; }
 
 extern "C" int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat) {
   return pb_rec_region_doubles(pb_rec_slots(total_points, ncat)) +
-         (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2);
+         (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2) +
+         (int64_t)PB_SUPER_STRIDE * (total_points / PB_SUPER_PTS + (int64_t)ncat + 2);
 }
 
 static int g_pb_fast_paths = 7;   // tgp_set_option("pairbin_fast_paths", bits): see PBParams::fast_paths
@@ -1742,13 +2071,50 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
   }
 
   if (split) {
-    // [0] pass A's work counter, [1] pass B's
+    // [0] pass A's work counter, [1] pass B's, [2] the super kernel's
     unsigned long long* ctr = reinterpret_cast<unsigned long long*>(work);
     P.rec_cnt = reinterpret_cast<int*>(work + 4);
     P.recs = reinterpret_cast<int4*>(work + 4 + rec_slots / 64);
     const int64_t per_round = (rec_slots < g_pb_rec_cap ? rec_slots : g_pb_rec_cap) / run;   // items
-    TGP_CUDA(cudaMemsetAsync(ctr, 0, 2 * sizeof(unsigned long long), st));
+    TGP_CUDA(cudaMemsetAsync(ctr, 0, 3 * sizeof(unsigned long long), st));
+    // super-chunk records (they follow the chunk records; the kernels find them from cat_off[ncat]) and the super
+    // kernel, which books the super pairs that the classification pass of every round skips
+    // kernel, which books the super pairs that the classification pass of every round skips.  Off when the staging
+    // buffer leaves no room for a warp histogram (the largest bin counts): then every super pair descends.
+    const int64_t nsf_max = max_cat_len / PB_SUPER_PTS;
+    const size_t per_warp_s = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0)) + 3 * PB_SUPER_PTS * 8;
+    int warps_s = (int)((budget - fixed - 64) / per_warp_s);
+    if (warps_s > PB_MAX_WARPS) warps_s = PB_MAX_WARPS;
+    const bool supers = nsf_max >= 2 && warps_s >= 1;
+    PBParams PS = P;
+    const int64_t super_items = nsf_max * ((nsf_max + 31) / 32) * ncat;
+    PS.items_per_cat = nsf_max;   // the super kernel's items of a catalogue: nsf_max rows x runs of 32 columns
+    PS.my_items = (super_items - tile_rank + tile_nranks - 1) / tile_nranks;
+    PS.counter = ctr + 2;
+    PS.warps = warps_s;
+    const size_t smem_s = fixed + (size_t)warps_s * per_warp_s + 64;
+    if (supers) {
+      pairbin_super_boxes_kernel<<<(unsigned)(nsf_max * ncat), PB_SUPER_PTS, 0, st>>>(
+          px, py, pk, pw, cat_off, ncat, nsf_max, const_cast<double*>(P.boxes));
+      TGP_LAUNCH_CHECK();
+    }
+    if (supers && PS.my_items > 0) {
+      static TgpPerDeviceOnce once_s[2];
+      const void* kern_s =
+          weighted ? (const void*)pairbin_super_kernel<true> : (const void*)pairbin_super_kernel<false>;
+      if (tgp_first_use_on_device(once_s[weighted ? 1 : 0]))
+        TGP_CUDA(cudaFuncSetAttribute(kern_s, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
+      int ctas_s = (int)((220 * 1024) / smem_s);
+      if (ctas_s > 2) ctas_s = 2;
+      if (ctas_s < 1) ctas_s = 1;
+      int64_t grid_s = tgp_cdiv(PS.my_items, warps_s);
+      if (grid_s > (int64_t)sms * ctas_s) grid_s = (int64_t)sms * ctas_s;
+      if (weighted) pairbin_super_kernel<true><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
+      else pairbin_super_kernel<false><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
+      TGP_LAUNCH_CHECK();
+    }
     PBParams PA = P;
+    PA.block_sums = supers ? 2 : 1;
     // pass A: warp histograms only (forward entries; bins x (count + sum [+ sum w])), as many warps per CTA as the
     // budget allows (up to 8): every nbins the residual kernel accepts runs
     const size_t per_warp_a = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0));
