@@ -6,7 +6,7 @@ NVFLAGS   := -O3 -std=c++17 -lineinfo $(ARCH) -Xcompiler -fPIC,-Wall,-Wno-unknow
 CSRC      := treegp_b200/csrc
 OBJDIR    := build
 LIB       := treegp_b200/libtreegp_b200.so
-SRCS      := kmat.cu dense.cu trsv.cu predict.cu pairbin.cu bootbin.cu microbench.cu hostrng.cu vcorr.cu collective.cu robustfit.cu selinv.cu
+SRCS      := kmat.cu dense.cu trsv.cu predict.cu pairbin.cu bootbin.cu microbench.cu hostrng.cu vcorr.cu collective.cu robustfit.cu selinv.cu batch.cu
 OBJS      := $(SRCS:%.cu=$(OBJDIR)/%.o)
 HDRS      := $(wildcard $(CSRC)/*.cuh) $(CSRC)/vk_tables.h include/treegp_b200.h
 

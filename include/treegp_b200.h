@@ -235,6 +235,36 @@ int tgp_predict_mean_trunc_multi(const double* Xs, int64_t M, const double* X, i
                                  const tgp_kernel_sum* k /*host*/, const double* alpha, int32_t r, double* mean,
                                  double* work, void* stream);
 
+/* ---- (2f) batches of independent problems ------------------------------------------------------------------------
+ * B problems, each with its own points, values, errors and kernel, in one call: every launch of the dense chain
+ * (K build, the panel steps of the Cholesky, the reductions) carries all of them, so that a batch of small problems
+ * takes about the launch latency of its largest one.  Problem b owns rows [off[b], off[b+1]) of the concatenated
+ * X (total x ndim), y, yerr2 and alpha; N_b = off[b+1] - off[b], 1 <= N_b <= TGP_BATCH_MAX_N.  ks[b] is its kernel (a
+ * one-term sum for a single kernel); one ndim for the whole batch.  off, soff and ks are HOST arrays; the entries
+ * stage them to the device themselves (stream-ordered allocation on `stream`).  Problems never influence one
+ * another: a problem's results are the same bit for bit whatever other problems share the batch and in whatever
+ * order.  The factorisation is always dense (no envelope).  Arguments are checked before any CUDA call. */
+#define TGP_BATCH_MAX_N 4096
+/* sum_b (N_b + 1) * ld_b doubles, ld_b = N_b rounded up to even; -1 for invalid B / off. */
+int64_t tgp_batch_work_doubles(const int64_t* off /*host*/, int32_t B);
+/* tgp_loglike_sum (dense, row_end == NULL) for every problem.  work: tgp_batch_work_doubles doubles, 16-byte aligned;
+ * problem b's (N_b + 1) x ld_b block starts at sum_{c < b} (N_c + 1) ld_c and holds on exit what tgp_loglike_sum
+ * leaves in its work (the factor in the lower triangle, L^-1 y in row N_b).  yerr2 is required (zeros for none).
+ * out: device double[3 B] = {logL, chi2, logdet} per problem, info: device int32[B], each with the meaning of
+ * tgp_loglike (logL = -inf for info > 0, NaN for info < 0).  want_alpha == 0: out, info and the factor equal
+ * tgp_loglike_sum on that problem alone bit for bit, alpha = L^-1 y.  want_alpha != 0: alpha = K^-1 y from a batched
+ * backward sweep (one CTA per problem), which may differ from the single call's sweep in the last bits, and
+ * chi2 = y . alpha. */
+int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, const int64_t* off /*host*/, int32_t B,
+                      const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, int want_alpha, double* out,
+                      int32_t* info, void* stream);
+/* mean rows [soff[b], soff[b+1]) = K_b(Xs_b, X_b) alpha_b, the full (untruncated) sum of tgp_predict_mean_sum summed
+ * in one pass over the training points (soff non-decreasing from 0: a problem may have no test points).  Equal bit
+ * for bit to tgp_predict_mean_sum wherever that call runs unsplit (N_b <= 1024 or many test points). */
+int tgp_predict_mean_batch(const double* Xs, const int64_t* soff /*host*/, const double* X, const int64_t* off /*host*/,
+                           int32_t B, const tgp_kernel_sum* ks /*host*/, const double* alpha, double* mean,
+                           void* stream);
+
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 
 /* mean[m] = sum_n K(Xs_m, X_n) alpha_n without materialising K(Xs, X).

@@ -10,6 +10,7 @@ from . import kernels as _k, log_likelihood as _ll, two_pcf as _tp, gp_interp as
 AnisotropicRBF, AnisotropicVonKarman, VonKarman, eval_kernel = (
     _k.AnisotropicRBF, _k.AnisotropicVonKarman, _k.VonKarman, _k.eval_kernel)
 GPInterpolation = _gi.GPInterpolation
+from .gp_batch import GPInterpolationBatch  # noqa: E402  (extension: many small problems per device call)
 # as in the reference, these two names are the classes (they shadow the sub-modules of the same name)
 log_likelihood, two_pcf = _ll.log_likelihood, _tp.two_pcf
 meanify = _mf.meanify
@@ -21,6 +22,7 @@ __version__ = "0.1.0"
 __all__ = [
     "__version__",
     "GPInterpolation",
+    "GPInterpolationBatch",
     "two_pcf",
     "log_likelihood",
     "AnisotropicRBF",

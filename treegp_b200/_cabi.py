@@ -25,6 +25,7 @@ class TgpKernel(ctypes.Structure):
 
 MAX_TERMS = 4   # TGP_MAX_TERMS
 MAX_RHS = 8     # TGP_MAX_RHS: outputs of the multi-output entries
+BATCH_MAX_N = 4096   # TGP_BATCH_MAX_N: points per problem of the batch entries
 
 
 class TgpKernelSum(ctypes.Structure):
@@ -75,6 +76,9 @@ SIGNATURES = {
     "tgp_loglike_grad_multi": [_vp, _vp, _i32, _vp, _i64, _ksp, _vp, _i64, _vp, _vp, _vp, _vp, _i64, _vp, _vp],
     "tgp_predict_mean_multi": [_vp, _i64, _vp, _i64, _ksp, _vp, _i32, _vp, _vp],
     "tgp_predict_mean_trunc_multi": [_vp, _i64, _vp, _i64, _ksp, _vp, _i32, _vp, _vp, _vp],
+    "tgp_batch_work_doubles": [_vp, _i32],
+    "tgp_loglike_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, ctypes.c_int, _vp, _vp, _vp],
+    "tgp_predict_mean_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -108,7 +112,7 @@ SIGNATURES = {
 _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctypes.c_int64,
              "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
              "tgp_loglike_grad_multi_work_doubles": ctypes.c_int64,
-             "tgp_predict_work_doubles": ctypes.c_int64,
+             "tgp_predict_work_doubles": ctypes.c_int64, "tgp_batch_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 
 _lib = None

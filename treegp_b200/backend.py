@@ -362,6 +362,93 @@ def loglike_grad_multi(X, Y, yerr2, kdesc, work=None, row_end=None):
     return out, info, alpha, work
 
 
+# ---- batches of independent problems (tgp_loglike_batch / tgp_predict_mean_batch) ----------------------------------
+def batch_offsets(sizes):
+    """Host int64 offsets [0, n_0, n_0 + n_1, ...] of problems with `sizes` points."""
+    return np.ascontiguousarray(np.concatenate([[0], np.cumsum(np.asarray(sizes, dtype=np.int64))]), dtype=np.int64)
+
+
+def batch_work_doubles(sizes):
+    """Workspace of tgp_loglike_batch: sum_b (N_b + 1) * ld_b doubles, ld_b = N_b rounded up to even."""
+    n = np.asarray(sizes, dtype=np.int64)
+    return int(np.sum((n + 1) * ((n + 1) & ~1)))
+
+
+def plan_batch_chunks(sizes, budget_bytes):
+    """Split problems with `sizes` points, in order, into consecutive chunks whose loglike_batch workspace fits
+    `budget_bytes`; a problem larger than the budget gets a chunk of its own.  Pure host function: returns a list of
+    (start, stop) index pairs covering range(len(sizes))."""
+    chunks, start, used = [], 0, 0
+    for b, n in enumerate(sizes):
+        need = 8 * batch_work_doubles([n])
+        if b > start and used + need > budget_bytes:
+            chunks.append((start, b))
+            start, used = b, 0
+        used += need
+    if len(sizes):
+        chunks.append((start, len(sizes)))
+    return chunks
+
+
+def _ksum_array(descs):
+    arr = (TgpKernelSum * len(descs))()
+    for b, d in enumerate(descs):
+        arr[b] = as_sum(d)
+    return arr
+
+
+def _check_batch_inputs(X, sizes, descs):
+    if len(sizes) != len(descs) or len(sizes) == 0:
+        raise ValueError("need one kernel descriptor per problem (%d sizes, %d descriptors)" % (len(sizes), len(descs)))
+    if X.shape[0] != int(np.sum(sizes)):
+        raise ValueError("X has %d rows but the problems have %d points" % (X.shape[0], int(np.sum(sizes))))
+    for d in descs:
+        _check_dims(d, X)
+
+
+def loglike_batch(X, y, yerr2, sizes, descs, want_alpha=False, budget_bytes=4 << 30):
+    """tgp_loglike_batch over B problems: X (sum N_b, ndim), y and yerr2 (sum N_b,) concatenated device tensors,
+    problem b owning `sizes[b]` consecutive rows; descs: B descriptors (TgpKernel or TgpKernelSum).  The problems are
+    put through in chunks whose workspace fits `budget_bytes` (plan_batch_chunks); the results do not depend on the
+    chunking.  Returns (out (B, 3) = logL, chi2, logdet per problem; info (B,); alpha (sum N_b,): K^-1 y with
+    want_alpha, else L^-1 y)."""
+    X = as_points(X)
+    sizes = [int(n) for n in sizes]
+    _check_batch_inputs(X, sizes, descs)
+    off = batch_offsets(sizes)
+    B = len(sizes)
+    out = torch.empty((B, 3), dtype=F64, device=X.device)
+    info = torch.empty(B, dtype=torch.int32, device=X.device)
+    alpha = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    lib = _cabi.load()
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes):
+        r0, r1 = int(off[b0]), int(off[b1])
+        o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
+        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        ks = _ksum_array(descs[b0:b1])
+        check(lib.tgp_loglike_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                    ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]), int(bool(want_alpha)),
+                                    _p(out[b0:b1]), _p(info[b0:b1]), _stream()), "tgp_loglike_batch")
+    return out, info, alpha
+
+
+def predict_mean_batch(Xs, ssizes, X, sizes, descs, alpha):
+    """tgp_predict_mean_batch: mean rows of problem b = K_b(Xs_b, X_b) alpha_b (the full sum), with Xs (sum M_b, ndim)
+    and X, alpha concatenated as for loglike_batch.  Returns the (sum M_b,) device tensor of means."""
+    Xs, X = as_points(Xs), as_points(X)
+    sizes, ssizes = [int(n) for n in sizes], [int(m) for m in ssizes]
+    _check_batch_inputs(X, sizes, descs)
+    if len(ssizes) != len(sizes) or Xs.shape[0] != int(np.sum(ssizes)):
+        raise ValueError("need one test-point count per problem, adding up to the rows of Xs")
+    _check_dims(descs[0], X, Xs)
+    mean = torch.empty(Xs.shape[0], dtype=F64, device=X.device)
+    soff, off, ks = batch_offsets(ssizes), batch_offsets(sizes), _ksum_array(descs)   # alive during the call
+    check(_cabi.load().tgp_predict_mean_batch(_p(Xs), _host_i64(soff), _p(X), _host_i64(off), len(sizes),
+                                              ctypes.cast(ks, ctypes.c_void_p), _p(alpha), _p(mean), _stream()),
+          "tgp_predict_mean_batch")
+    return mean
+
+
 TRUNC_MIN_M, TRUNC_MIN_N = 16384, 2048   # below this the plain kernel is launch-bound anyway
 
 

@@ -23,6 +23,7 @@
 #include <atomic>
 #include "tgp_common.cuh"
 #include "profile_policy.cuh"
+#include "batch.cuh"
 
 // ============================================================================================
 // gemm_nt_sub
@@ -71,17 +72,17 @@ __device__ __forceinline__ void load_operand_stage(double* smem, const double* _
 //   <128, 2, 4, 1>: 128 x 128 tile, warp tile 64 x 32, one CTA per SM (largest operand reuse);
 //   < 64, 4, 2, 2>: 128 x  64 tile, warp tile 32 x 32, two CTAs per SM so that the epilogue (C read-modify-
 //                   write) and the pipeline fill of one CTA hide under the DMMA work of the other.
-template <int BN_, int WARPS_M, int WARPS_N, int MIN_CTAS>
-__global__ void __launch_bounds__(GEMM_THREADS, MIN_CTAS)
-gemm_nt_sub_kernel(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
-                   const double* __restrict__ A, int64_t lda, const double* __restrict__ B, int64_t ldb,
-                   int64_t Kd, int lower_only) {
+// The CTA tile whose top-left corner is (m0, n0).
+template <int BN_, int WARPS_M, int WARPS_N>
+__device__ __forceinline__ void gemm_nt_sub_tile(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
+                                                 const double* __restrict__ A, int64_t lda,
+                                                 const double* __restrict__ B, int64_t ldb, int64_t Kd,
+                                                 int lower_only, const int64_t m0, const int64_t n0) {
   constexpr int WM = BM / WARPS_M, WN = BN_ / WARPS_N;   // warp tile
   constexpr int MB = WM / 8, NBK = WN / 8;                // 8x8 blocks per warp tile
   constexpr int STAGE_D = (BM + BN_) * BK;
   static_assert(WARPS_M * WARPS_N == 8, "8 warps");
   extern __shared__ __align__(16) double gsm[];
-  const int64_t m0 = (int64_t)blockIdx.y * BM, n0 = (int64_t)blockIdx.x * BN_;
   if (lower_only && n0 > m0 + BM - 1) return;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int wm0 = (warp / WARPS_N) * WM, wn0 = (warp % WARPS_N) * WN;
@@ -160,6 +161,15 @@ gemm_nt_sub_kernel(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
       }
     }
   }
+}
+
+template <int BN_, int WARPS_M, int WARPS_N, int MIN_CTAS>
+__global__ void __launch_bounds__(GEMM_THREADS, MIN_CTAS)
+gemm_nt_sub_kernel(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
+                   const double* __restrict__ A, int64_t lda, const double* __restrict__ B, int64_t ldb,
+                   int64_t Kd, int lower_only) {
+  gemm_nt_sub_tile<BN_, WARPS_M, WARPS_N>(C, M, Nc, ldc, A, lda, B, ldb, Kd, lower_only, (int64_t)blockIdx.y * BM,
+                                          (int64_t)blockIdx.x * BN_);
 }
 
 static int g_lookahead = 1;  // 0 disables the two-stream look-ahead Cholesky driver
@@ -533,17 +543,17 @@ extern "C" int tgp_debug_potf2_cycles(unsigned long long* host4) {
 #define PL_T(i)
 #endif
 
-__global__ void __launch_bounds__(PL_THREADS, 2)
-panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, int j, int32_t* __restrict__ info,
-                  int64_t goff, unsigned slot, unsigned epoch) {
+// CTA number `cta` of one launch (flag: the launch's inter-CTA flag word).
+__device__ __forceinline__ void panel_left_body(double* __restrict__ Akk, int64_t ld, int w, int64_t below, int j,
+                                                int32_t* __restrict__ info, int64_t goff, unsigned* flag,
+                                                unsigned epoch, const unsigned cta) {
   extern __shared__ __align__(16) double psm[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int ndiag = (w + NB - 1) / NB;
   const int c0 = j * NB;
   const int nbj = (w - c0 < NB) ? (w - c0) : NB;
-  unsigned* flag = &g_panel_flags[slot];
 
-  if (blockIdx.x == 0) {
+  if (cta == 0) {
     double* S = psm;                       // NB x NB_PITCH
     double* rdiag = psm + NB * NB_PITCH;
     double* D = Akk + (int64_t)c0 * ld + c0;
@@ -561,7 +571,7 @@ panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, in
     return;
   }
 
-  const int rb = j + blockIdx.x;           // row block: < ndiag inside D, else among the rows below
+  const int rb = j + cta;                  // row block: < ndiag inside D, else among the rows below
   const bool in_diag = rb < ndiag;
   int64_t r0;
   int nrows;
@@ -576,7 +586,7 @@ panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, in
   const int g = lane >> 2, t = lane & 3;
   const int wm0 = (warp >> 2) * 32, wn0 = (warp & 3) * 16;   // warp tile 32 x 16 of the 64 x 64 block
 #ifdef TGP_PANEL_TIMING
-  const bool stamp = blockIdx.x == 1;
+  const bool stamp = cta == 1;
 #undef PL_T
 #define PL_T(i) if (stamp) pl_stamp(i)
 #endif
@@ -815,6 +825,12 @@ panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, in
     if (r < nrows && c < nbj) Akk[(r0 + r) * ld + c0 + c] = Ts[r * PL_P + c];
   }
   PL_T(14);
+}
+
+__global__ void __launch_bounds__(PL_THREADS, 2)
+panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, int j, int32_t* __restrict__ info,
+                  int64_t goff, unsigned slot, unsigned epoch) {
+  panel_left_body(Akk, ld, w, below, j, info, goff, &g_panel_flags[slot], epoch, blockIdx.x);
 }
 
 
@@ -1283,9 +1299,9 @@ extern "C" int tgp_potrs_vec(const double* L, int64_t N, int64_t ld, double* b, 
 // Reductions: log-determinant, chi2 = y . alpha, final log-likelihood.
 // ============================================================================================
 // out[0] = sum 2 log L_ii ; out[1] = y . alpha (if given).  Single CTA, deterministic order.
-__global__ void __launch_bounds__(1024)
-logdet_chi2_kernel(const double* __restrict__ L, int64_t N, int64_t ld, const double* __restrict__ y,
-                   const double* __restrict__ alpha, double* __restrict__ out) {
+__device__ __forceinline__ void logdet_chi2_body(const double* __restrict__ L, int64_t N, int64_t ld,
+                                                 const double* __restrict__ y, const double* __restrict__ alpha,
+                                                 double* __restrict__ out) {
   __shared__ double s0[32], s1[32];
   double a = 0.0, c = 0.0;
   for (int64_t i = threadIdx.x; i < N; i += blockDim.x) {
@@ -1314,6 +1330,11 @@ logdet_chi2_kernel(const double* __restrict__ L, int64_t N, int64_t ld, const do
     }
   }
 }
+__global__ void __launch_bounds__(1024)
+logdet_chi2_kernel(const double* __restrict__ L, int64_t N, int64_t ld, const double* __restrict__ y,
+                   const double* __restrict__ alpha, double* __restrict__ out) {
+  logdet_chi2_body(L, N, ld, y, alpha, out);
+}
 
 extern "C" int tgp_logdet_chi2(const double* L, int64_t N, int64_t ld, const double* y, const double* alpha,
                                double* out, void* stream) {
@@ -1325,7 +1346,8 @@ extern "C" int tgp_logdet_chi2(const double* L, int64_t N, int64_t ld, const dou
 }
 
 // out = {logL, chi2, logdet}; tmp = {logdet, chi2}.
-__global__ void loglike_finish_kernel(const double* tmp, int64_t N, const int32_t* __restrict__ info, double* out) {
+__device__ __forceinline__ void loglike_finish_body(const double* tmp, int64_t N, const int32_t* __restrict__ info,
+                                                    double* out) {
   const double logdet = tmp[0], chi2 = tmp[1];
   double ll = -0.5 * chi2 - 0.5 * (double)N * log(2.0 * TGP_PI) - 0.5 * logdet;
   // info > 0: leading minor not positive definite -> -inf (log_likelihood.py:38-39).  info < 0: an internal
@@ -1336,10 +1358,12 @@ __global__ void loglike_finish_kernel(const double* tmp, int64_t N, const int32_
   out[1] = chi2;
   out[2] = logdet;
 }
+__global__ void loglike_finish_kernel(const double* tmp, int64_t N, const int32_t* __restrict__ info, double* out) {
+  loglike_finish_body(tmp, N, info, out);
+}
 
 // chi2 = ||w||^2 with w = L^-1 y (forward sweep only) -- y^T K^-1 y without the backward solve.
-__global__ void __launch_bounds__(1024)
-sumsq_kernel(const double* __restrict__ w, int64_t N, double* __restrict__ out1) {
+__device__ __forceinline__ void sumsq_body(const double* __restrict__ w, int64_t N, double* __restrict__ out1) {
   __shared__ double s0[32];
   double a = 0.0;
   for (int64_t i = threadIdx.x; i < N; i += blockDim.x) a = fma(w[i], w[i], a);
@@ -1354,6 +1378,10 @@ sumsq_kernel(const double* __restrict__ w, int64_t N, double* __restrict__ out1)
     for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
     if (lane == 0) *out1 = a;
   }
+}
+__global__ void __launch_bounds__(1024)
+sumsq_kernel(const double* __restrict__ w, int64_t N, double* __restrict__ out1) {
+  sumsq_body(w, N, out1);
 }
 
 static int loglike_args(const double* X, const double* y, int64_t N, const double* work, const double* alpha,
@@ -1532,6 +1560,111 @@ extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, co
   loglike_multi_finish_kernel<<<1, 1024, 0, st>>>(work, N, ld, Y, r, rows, want_alpha, info, out);
   TGP_LAUNCH_CHECK();
   multi_transpose_kernel<<<tg, 256, 0, st>>>(alpha, r, rows, ld, N, 0);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// ============================================================================================
+// Batches of independent problems (tgp_loglike_batch).  The schedule of potrf_rec with y riding along as row N, run
+// once over the panel steps of the largest problem: every launch covers each problem that still has columns at that
+// step (CTAs of the others exit), and each CTA runs the body of the single-problem kernel on its problem's block.
+// For N >= 3 OB the single call takes the look-ahead driver, whose U1 / U2 updates split the same K = OB update by
+// columns: per element the same DMMA chain, so the factor is the same bit for bit.
+// ============================================================================================
+// grid: (problem, CTA of the panel launch); the CTAs 0 of all problems are dispatched before any CTA that waits.
+__global__ void __launch_bounds__(PL_THREADS, 2)
+panel_left_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int j, int32_t* __restrict__ info,
+                        unsigned* __restrict__ flags, unsigned epoch) {
+  const int b = blockIdx.x;
+  const int64_t N = pr[b].N;
+  if (k >= N) return;
+  const int w = (int)(N - k < OB ? N - k : OB);
+  const int ndiag = (w + NB - 1) / NB;
+  if (j >= ndiag) return;
+  const int64_t below = N - k - w + 1;
+  if ((int64_t)blockIdx.y >= (ndiag - j) + (below + NB - 1) / NB) return;
+  const int64_t ld = pr[b].ld;
+  panel_left_body(pr[b].A + k * ld + k, ld, w, below, j, info + b, k, flags + b, epoch, blockIdx.y);
+}
+
+// The trailing update of outer step k: C (rest + 1 x rest) -= L21 L21^T (lower), the y row included.
+// grid: (problem, row tile * tiles_n + column tile).
+__global__ void __launch_bounds__(GEMM_THREADS, 2)
+gemm_trail_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int tiles_n) {
+  const int b = blockIdx.x;
+  const int64_t N = pr[b].N;
+  const int64_t w = N - k < OB ? N - k : OB, rest = N - k - w;
+  if (rest <= 0) return;
+  const int64_t m0 = (int64_t)(blockIdx.y / tiles_n) * BM, n0 = (int64_t)(blockIdx.y % tiles_n) * 64;
+  if (m0 >= rest + 1 || n0 >= rest) return;
+  const int64_t ld = pr[b].ld;
+  double* Ark = pr[b].A + (k + w) * ld + k;
+  gemm_nt_sub_tile<64, 4, 2>(Ark + w, rest + 1, rest, ld, Ark, ld, Ark, ld, w, 1, m0, n0);
+}
+
+int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, int32_t* info, unsigned* flags,
+                         cudaStream_t st) {
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once)) {
+    constexpr int GSMEM = STAGES * (BM + 64) * BK * 8;
+    TGP_CUDA(cudaFuncSetAttribute(panel_left_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PL_SMEM));
+    TGP_CUDA(cudaFuncSetAttribute(panel_left_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+    TGP_CUDA(cudaFuncSetAttribute(gemm_trail_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM));
+    TGP_CUDA(cudaFuncSetAttribute(gemm_trail_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+  }
+  TGP_CUDA(cudaMemsetAsync(info, 0, sizeof(int32_t) * B, st));
+  int64_t nmax = 0;
+  for (int32_t b = 0; b < B; ++b) nmax = Nh[b] > nmax ? Nh[b] : nmax;
+  unsigned epoch = 0;   // the flags start at 0 and every panel launch of this call takes the next epoch
+  for (int64_t k = 0; k < nmax; k += OB) {
+    const int64_t wmax = nmax - k < OB ? nmax - k : OB;
+    for (int j = 0; j < (int)tgp_cdiv(wmax, NB); ++j) {
+      int64_t ctas = 0;   // the largest launch of a problem at this step
+      for (int32_t b = 0; b < B; ++b) {
+        if (Nh[b] <= k) continue;
+        const int64_t w = Nh[b] - k < OB ? Nh[b] - k : OB, ndiag = tgp_cdiv(w, NB);
+        if (j >= ndiag) continue;
+        const int64_t c = (ndiag - j) + tgp_cdiv(Nh[b] - k - w + 1, NB);
+        ctas = c > ctas ? c : ctas;
+      }
+      panel_left_batch_kernel<<<dim3((unsigned)B, (unsigned)ctas), PL_THREADS, PL_SMEM, st>>>(pr, k, j, info, flags,
+                                                                                             ++epoch);
+      TGP_LAUNCH_CHECK();
+    }
+    const int64_t rest = nmax - k - wmax;   // the largest trailing update belongs to the largest problem
+    if (rest > 0) {
+      const int tiles_n = (int)tgp_cdiv(rest, 64);
+      const int64_t tiles = tgp_cdiv(rest + 1, BM) * tiles_n;
+      gemm_trail_batch_kernel<<<dim3((unsigned)B, (unsigned)tiles), GEMM_THREADS, STAGES * (BM + 64) * BK * 8, st>>>(
+          pr, k, tiles_n);
+      TGP_LAUNCH_CHECK();
+    }
+  }
+  return TGP_OK;
+}
+
+// One CTA per problem: the reductions of loglike_after_build and loglike_finish_kernel, same bodies, same order.
+__global__ void __launch_bounds__(1024)
+loglike_batch_finish_kernel(const TgpBatchProb* __restrict__ pr, int want_alpha, const int32_t* __restrict__ info,
+                            double* __restrict__ out) {
+  __shared__ double tmp[2];   // {logdet, chi2}
+  const TgpBatchProb& p = pr[blockIdx.x];
+  if (want_alpha) {
+    logdet_chi2_body(p.A, p.N, p.ld, p.y, p.alpha, tmp);   // chi2 = y . alpha
+  } else {
+    logdet_chi2_body(p.A, p.N, p.ld, nullptr, nullptr, tmp);
+    __syncthreads();
+    sumsq_body(p.alpha, p.N, tmp + 1);                      // chi2 = ||L^-1 y||^2
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) loglike_finish_body(tmp, p.N, info + blockIdx.x, out + 3 * (int64_t)blockIdx.x);
+}
+
+int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int want_alpha, const int32_t* info, double* out,
+                             cudaStream_t st) {
+  loglike_batch_finish_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, want_alpha, info, out);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

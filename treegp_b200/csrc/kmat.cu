@@ -15,6 +15,7 @@
 #include <string.h>
 #include "tgp_common.cuh"
 #include "profile_policy.cuh"
+#include "batch.cuh"
 
 // ---- error state / misc host helpers --------------------------------------------------------
 static thread_local char g_err[512] = "";
@@ -64,18 +65,17 @@ __device__ __forceinline__ void store2(double* p, double a, double b, bool vec, 
   }
 }
 
-// Symmetric build.  Grid: one CTA per lower-triangular tile pair (I >= J), linearised.
+// Symmetric build of the lower-triangular tile pair number t (I >= J, linearised).
 template <class P>
-__global__ void __launch_bounds__(KT_THREADS)
-kmat_sym_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ diag_add,
-                double* __restrict__ out, int64_t ld, int lower_only, int vec_ok,
-                const double* __restrict__ phi_g) {
+__device__ __forceinline__ void kmat_sym_tile(const double* __restrict__ X, int64_t N, const P& prof,
+                                              const double* __restrict__ diag_add, double* __restrict__ out,
+                                              int64_t ld, int lower_only, int vec_ok,
+                                              const double* __restrict__ phi_g, const int64_t t) {
   __shared__ double xr[KT], yr[KT], xc[KT], yc[KT];
   __shared__ double tile[KT * KT_PITCH];
   __shared__ double phi_s[P::kPhiSize];
 
   // linear tile id -> (I, J), I >= J
-  const int64_t t = blockIdx.x;
   int64_t I = (int64_t)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
   while (I * (I + 1) / 2 > t) --I;
   while ((I + 1) * (I + 2) / 2 <= t) ++I;
@@ -148,6 +148,15 @@ kmat_sym_kernel(const double* __restrict__ X, int64_t N, P prof, const double* _
       if (r0 + lane + 32 < N) dst[lane + 32] = b;
     }
   }
+}
+
+// Grid: one CTA per lower-triangular tile pair.
+template <class P>
+__global__ void __launch_bounds__(KT_THREADS)
+kmat_sym_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ diag_add,
+                double* __restrict__ out, int64_t ld, int lower_only, int vec_ok,
+                const double* __restrict__ phi_g) {
+  kmat_sym_tile(X, N, prof, diag_add, out, ld, lower_only, vec_ok, phi_g, (int64_t)blockIdx.x);
 }
 
 // Rectangular build K(Xs, X): rows = test points, columns = training points.
@@ -259,6 +268,36 @@ extern "C" int tgp_kmat_cross_sum(const double* Xs, int64_t M, const double* X, 
   TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
   kmat_cross_kernel<SumProfile><<<grid, KT_THREADS, 0, (cudaStream_t)stream>>>(
       Xs, M, X, N, SumProfile{make_ksumdesc(k)}, out, ld, vec_ok, tgp_phi_device());
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// ---- batches of independent problems (tgp_loglike_batch) ---------------------------------------------------------
+// K(X_b, X_b) + diag(yerr2_b), lower triangle, into problem b's block of the batch workspace.  Grid: (problems of
+// this profile class, tiles of the largest of them); each CTA runs the tile body of the single build with the
+// problem's descriptor, so every problem gets the single call's matrix bit for bit.
+template <class P>
+__global__ void __launch_bounds__(KT_THREADS)
+kmat_sym_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* __restrict__ kd,
+                      const int32_t* __restrict__ list, const double* __restrict__ phi_g) {
+  const int b = list[blockIdx.x];
+  const int64_t N = pr[b].N, nt = (N + KT - 1) / KT;
+  if ((int64_t)blockIdx.y >= nt * (nt + 1) / 2) return;
+  const P prof = tgp_batch_profile<P>(kd[b]);
+  kmat_sym_tile(pr[b].X, N, prof, pr[b].yerr2, pr[b].A, pr[b].ld, /*lower_only=*/1, /*vec_ok=*/1, phi_g,
+                (int64_t)blockIdx.y);
+}
+
+int tgp_batch_kmat_sym(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
+                       int64_t max_n, cudaStream_t st) {
+  const int64_t nt = tgp_cdiv(max_n, KT);
+  const dim3 grid((unsigned)count, (unsigned)(nt * (nt + 1) / 2));
+  const double* phi = tgp_phi_device();
+  if (cls == TGP_BATCH_SUM) {
+    kmat_sym_batch_kernel<SumProfile><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi);
+  } else {
+    TGP_FAMILY_SWITCH(cls, (kmat_sym_batch_kernel<FamilyProfile<FAM>><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi)));
+  }
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

@@ -6,6 +6,7 @@
 // coordinates and alpha stream through shared memory, and only M doubles are written.
 #include "tgp_common.cuh"
 #include "profile_policy.cuh"
+#include "batch.cuh"
 
 constexpr int PM_THREADS = 256;   // test points per CTA
 constexpr int PM_TILE = 1024;     // training points per shared-memory tile
@@ -16,11 +17,31 @@ constexpr int PM_TILE = 1024;     // training points per shared-memory tile
 // Several outputs (P = MultiOut<..., R>): alpha and mean are row-major (N, r) and (M, r); each thread keeps R pairs of
 // accumulators, evaluates every pair's profile once and applies it to all columns -- each column in the order of the
 // single-output kernel.  The tile shrinks with R so that the staged alpha stays at 16 KB.
-template <class P>
+// BATCH (tgp_predict_mean_batch): grid (problems of one profile class, test-point blocks of the largest of them); the
+// problem's slices and descriptor replace the arguments, and every CTA sums all training tiles of its problem in order
+// (one split): the single call's sum whenever that call runs unsplit, independent of the other problems.
+template <class P, bool BATCH = false>
 __global__ void __launch_bounds__(PM_THREADS)
 predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
                     P prof, const double* __restrict__ alpha, double* __restrict__ mean,
-                    const double* __restrict__ phi_g) {
+                    const double* __restrict__ phi_g, const TgpBatchProb* __restrict__ pr = nullptr,
+                    const KSumDesc* __restrict__ kd = nullptr, const int32_t* __restrict__ list = nullptr) {
+  unsigned bx = blockIdx.x, by = blockIdx.y;
+  int nsplit = gridDim.y;
+  if constexpr (BATCH) {
+    const int b = list[blockIdx.x];
+    M = pr[b].M;
+    if ((int64_t)blockIdx.y * PM_THREADS >= M) return;
+    Xs = pr[b].Xs;
+    X = pr[b].X;
+    N = pr[b].N;
+    alpha = pr[b].alpha;
+    mean = pr[b].mean;
+    prof = tgp_batch_profile<P>(kd[b]);
+    bx = blockIdx.y;
+    by = 0;
+    nsplit = 1;
+  }
   constexpr int R = OutputsOf<P>::kR;
   constexpr int TILE = R == 1 ? PM_TILE : 2048 / R;
   __shared__ double2 pxy[TILE];
@@ -28,17 +49,16 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
   __shared__ double phi_s[P::kPhiSize];
   const int tid = threadIdx.x;
   if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
-  const int64_t m = (int64_t)blockIdx.x * PM_THREADS + tid;
+  const int64_t m = (int64_t)bx * PM_THREADS + tid;
   const bool live = m < M;
   const double sx = live ? Xs[m * prof.desc.ndim] : 0.0;
   const double sy = (live && prof.desc.ndim == 2) ? Xs[m * 2 + 1] : 0.0;
-  const int nsplit = gridDim.y;
   const int64_t ntile = (N + TILE - 1) / TILE;
   double acc0 = 0.0, acc1 = 0.0;
   double accm0[R], accm1[R];
 #pragma unroll
   for (int c = 0; c < R; ++c) accm0[c] = accm1[c] = 0.0;
-  for (int64_t tl = blockIdx.y; tl < ntile; tl += nsplit) {
+  for (int64_t tl = by; tl < ntile; tl += nsplit) {
     const int64_t n0 = tl * TILE;
     __syncthreads();
     for (int i = tid; i < TILE; i += PM_THREADS) {
@@ -128,6 +148,23 @@ extern "C" int tgp_predict_mean_sum(const double* Xs, int64_t M, const double* X
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   if (k->nterms == 1) return tgp_predict_mean(Xs, M, X, N, &k->term[0], alpha, mean, stream);
   return predict_mean_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, alpha, mean, stream);
+}
+
+int tgp_batch_predict_mean(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
+                           int64_t max_m, cudaStream_t st) {
+  const int64_t gy = tgp_cdiv(max_m, PM_THREADS);
+  TGP_CHECK_ARG(gy <= 65535, "too many test points in one problem (at most 65535 * 256)");
+  const dim3 grid((unsigned)count, (unsigned)gy);
+  const double* phi = tgp_phi_device();
+  if (cls == TGP_BATCH_SUM) {
+    predict_mean_kernel<SumProfile, true><<<grid, PM_THREADS, 0, st>>>(nullptr, 0, nullptr, 0, SumProfile{}, nullptr,
+                                                                      nullptr, phi, pr, kd, list);
+  } else {
+    TGP_FAMILY_SWITCH(cls, (predict_mean_kernel<FamilyProfile<FAM>, true><<<grid, PM_THREADS, 0, st>>>(
+                               nullptr, 0, nullptr, 0, FamilyProfile<FAM>{}, nullptr, nullptr, phi, pr, kd, list)));
+  }
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
