@@ -475,9 +475,8 @@ int tgp_pairbin_tile(void);
  * point on the super-chunk's sorted copy.  The slots are disjoint.  Synchronous. */
 int tgp_pairbin_stats(unsigned long long* host8 /*host*/, int reset);
 
-/* Tuning knobs for experiments (not needed for normal use).  "trsv_cluster": thread-block cluster size of the
- * triangular sweeps (-1 automatic, 1 = no clusters, 2 / 4 / 8).  "gemm_config": -1 automatic,
- * 0 = 128x128 CTA tile (1 CTA/SM), 1 = 128x64 CTA tile (2 CTAs/SM); "potrf_fused": 0 = unfused panel chain;
+/* Test and measurement switches of the pair counts (tgp_pairbin_*, tgp_bootbin_twod), not needed for normal use.
+ * Any other name is rejected with TGP_ERR_INVALID ("unknown option").
  * "pairbin_block_sums": 0 = every pair of every in-range block is evaluated individually (no block forms);
  * "pairbin_fast_paths": bit mask, default all on; bit 0 = short-cut dispatch of one-axis blocks that fit the open
  * bin window, bit 1 = 2 x 2-window blocks take their marginal sums from rank queries, bit 2 = the pair-by-pair kernel

@@ -55,6 +55,22 @@ def test_invalid_arguments_are_rejected_without_a_gpu():
     assert lib.tgp_predict_var_env(A16, 4, A16, 1000, ctypes.byref(ok), A16, 1000, None, 2, A16, 128, A16, None) == -1
 
 
+def test_set_option_knows_only_the_pair_count_switches():
+    """The four switches of the pair counts are accepted (and set back to their defaults); any other name is an
+    unknown option, including the retired Cholesky, GEMM and sweep selections."""
+    from treegp_b200 import _cabi
+
+    lib = _cabi.load()
+    for name in ("potrf_fused", "potrf_lookahead", "potrf_ob", "potrf_env_lookahead", "gemm_config", "trsv_cluster",
+                 "no_such_option"):
+        assert lib.tgp_set_option(name.encode(), 0) == -1, name
+        assert b"unknown option" in lib.tgp_last_error()
+    assert lib.tgp_set_option(None, 0) == -1
+    for name, default in (("pairbin_block_sums", 1), ("pairbin_fast_paths", 7), ("pairbin_record_cap", 0),
+                          ("bootbin_paths", 15)):
+        assert lib.tgp_set_option(name.encode(), default) == 0, name
+
+
 def test_product_path_does_not_import_the_oracle():
     """The oracle is test infrastructure: nothing under treegp_b200/ may reference it."""
     pkg = os.path.join(ROOT, "treegp_b200")

@@ -72,6 +72,34 @@ def test_potrf_env_and_loglike_env_equal_the_dense_calls(gpu_ready, case, n, fie
     np.testing.assert_allclose(got, alpha, rtol=0, atol=1e-8 * np.max(np.abs(alpha)))
 
 
+def test_potrf_env_carries_extra_rows_as_the_dense_call(gpu_ready):
+    """tgp_potrf_env with right-hand-side rows below the matrix (nrows > 0): the factor and the rows L^-1 y equal
+    those of tgp_potrf_rows on the same sorted problem.  The rows ride inside the panel solves of the block columns
+    whose envelope reaches N and take their own solve and update in the others."""
+    import torch
+    from treegp_b200 import _cabi, backend
+
+    n, r = 6000, 3
+    X, y, e2, desc, plan = _problem("rbf2", n, 260.0)
+    o, re = plan["order"], plan["row_end"]
+    assert re[0] < n and re[-1] == n
+    A = backend.alloc_matrix(n + r, n)
+    backend.kmat_sym(backend.as_points(X)[o].contiguous(), desc, backend.to_device(e2)[o].contiguous(), out=A,
+                     lower_only=True)
+    A[n:, :n] = backend.to_device(np.random.default_rng(5).normal(size=(r, n)))
+    B = A.clone()
+    lib = _cabi.load()
+    ia, ib = (torch.ones(1, dtype=torch.int32, device=A.device) for _ in range(2))
+    assert lib.tgp_potrf_rows(backend._p(A), n, A.stride(0), r, backend._p(ia), backend._stream()) == 0
+    assert lib.tgp_potrf_env(backend._p(B), n, B.stride(0), backend._host_i64(re), len(re), r, backend._p(ib),
+                             backend._stream()) == 0
+    assert int(ia.item()) == 0 and int(ib.item()) == 0
+    La, Lb = np.tril(A[:n, :n].cpu().numpy()), np.tril(B[:n, :n].cpu().numpy())
+    assert np.max(np.abs(La - Lb)) <= 1e-11 * np.max(np.abs(La))
+    Wa, Wb = A[n:, :n].cpu().numpy(), B[n:, :n].cpu().numpy()
+    assert np.max(np.abs(Wa - Wb)) <= 1e-11 * np.max(np.abs(Wa))
+
+
 def test_envelope_reports_a_matrix_that_is_not_positive_definite(gpu_ready):
     """info is the failing leading minor, as from the dense call, and logL is -inf (log_likelihood.py:38-39)."""
     from treegp_b200 import backend

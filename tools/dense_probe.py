@@ -12,8 +12,6 @@ def timed(fn, reps=3):
         a.record(); fn(); b.record(); torch.cuda.synchronize(); ts.append(a.elapsed_time(b) * 1e-3)
     return min(ts)
 
-backend.set_option("gemm_config", int(os.environ.get("G_CFG", "-1")))
-backend.set_option("potrf_ob", int(os.environ.get("P_OB", "0")))
 for (m, n, k, low) in [(20480, 20480, 512, 1), (20480, 20480, 512, 0), (40960, 512, 64, 0), (8192, 8192, 512, 1), (30000, 448, 64, 0)]:
     C = torch.zeros((m, backend.even(n)), dtype=torch.float64, device="cuda")
     A = torch.randn((m, k), dtype=torch.float64, device="cuda")

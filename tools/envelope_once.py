@@ -13,8 +13,6 @@ from treegp_b200 import backend  # noqa: E402
 from treegp_b200.kernels import lower_kernel  # noqa: E402
 
 n = int(os.environ.get("PN", "40000"))
-if os.environ.get("TRSV_NOCLUSTER"):     # ncu cannot replay the cluster + cooperative launch of the sweeps
-    backend.set_option("trsv_cluster", 1)
 X, _, kstr, _, _, noise, _ = bench.gp_problem(n, 16)
 desc = lower_kernel(treegp.eval_kernel(kstr), 2)
 Xd = backend.as_points(X)

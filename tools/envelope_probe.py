@@ -73,8 +73,6 @@ def probe(name, X, kstr, noise):
 
 
 def main():
-    if os.environ.get("ENV_LA") is not None:
-        backend.set_option("potrf_env_lookahead", int(os.environ["ENV_LA"]))
     X, _, kstr, _, _, noise, _ = bench.gp_problem(int(os.environ.get("PN", "40000")), 16)
     probe("configs[2]", X, kstr, noise)
     rng = np.random.default_rng(7)

@@ -11,8 +11,6 @@ vp, i64 = ctypes.c_void_p, ctypes.c_int64
 lib.tgp_trsv_only.argtypes = [vp, i64, i64, vp, ctypes.c_int, vp]
 lib.tgp_device_error.argtypes = [ctypes.c_int]
 n, which = int(sys.argv[1]), int(sys.argv[2])
-if len(sys.argv) > 3:
-    lib.tgp_set_option(b"trsv_cluster", int(sys.argv[3]))
 ws = torch.randn((n, n + (n & 1)), dtype=torch.float64, device="cuda") * (0.5 / np.sqrt(n))
 ws[:, :n].diagonal().fill_(1.5)
 b = torch.randn(n, dtype=torch.float64, device="cuda")

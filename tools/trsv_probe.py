@@ -1,8 +1,6 @@
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from treegp_b200 import backend
-if "TGP_TRSV_CLUSTER" in os.environ:   # 1 = no thread-block clusters (ncu cannot replay cluster + cooperative launches)
-    backend.set_option("trsv_cluster", int(os.environ["TGP_TRSV_CLUSTER"]))
 def timed(fn, reps=3):
     fn(); torch.cuda.synchronize(); ts = []
     for _ in range(reps):

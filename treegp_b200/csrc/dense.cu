@@ -68,10 +68,9 @@ __device__ __forceinline__ void load_operand_stage(double* smem, const double* _
 }
 
 // C (M x Nc) -= A (M x Kd) * B^T (Nc x Kd).  lower_only: skip tiles above the diagonal and mask n > m.
-// CTA tile BM x BN_, 8 warps arranged WARPS_M x WARPS_N.  Two configurations are instantiated:
-//   <128, 2, 4, 1>: 128 x 128 tile, warp tile 64 x 32, one CTA per SM (largest operand reuse);
-//   < 64, 4, 2, 2>: 128 x  64 tile, warp tile 32 x 32, two CTAs per SM so that the epilogue (C read-modify-
-//                   write) and the pipeline fill of one CTA hide under the DMMA work of the other.
+// CTA tile BM x BN_, 8 warps arranged WARPS_M x WARPS_N.  The launches use <64, 4, 2, 2>: 128 x 64 tile, warp tile
+// 32 x 32, two CTAs per SM so that the epilogue (C read-modify-write) and the pipeline fill of one CTA hide under the
+// DMMA work of the other.
 // The CTA tile whose top-left corner is (m0, n0).
 template <int BN_, int WARPS_M, int WARPS_N>
 __device__ __forceinline__ void gemm_nt_sub_tile(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
@@ -172,65 +171,42 @@ gemm_nt_sub_kernel(double* __restrict__ C, int64_t M, int64_t Nc, int64_t ldc,
                                           (int64_t)blockIdx.x * BN_);
 }
 
-static int g_lookahead = 1;  // 0 disables the two-stream look-ahead Cholesky driver
-static int g_ob_large = 0;   // outer block of the look-ahead driver: 0 = automatic, else a multiple of 512 (option "potrf_ob")
-static int g_fused_panel = 1;   // option "potrf_fused": 0 = the potf2 / trsm_panel / gemm chain per 64 columns
-static int g_env_lookahead = 1;   // option "potrf_env_lookahead": 0 = the sequential envelope driver, 2 = see there
-static int g_gemm_config = -1;  // -1: pick by shape; 0: 128x128; 1: 128x64 (tgp_set_option for experiments)
-
-template <int BN_, int WARPS_M, int WARPS_N, int MIN_CTAS>
-static int gemm_launch_cfg(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
-                           const double* B, int64_t ldb, int64_t Kd, int lower_only, cudaStream_t st) {
-  constexpr int SMEM = STAGES * (BM + BN_) * BK * 8;
-  static TgpPerDeviceOnce attr_once;
-  if (tgp_first_use_on_device(attr_once)) {
-    TGP_CUDA(cudaFuncSetAttribute(gemm_nt_sub_kernel<BN_, WARPS_M, WARPS_N, MIN_CTAS>,
-                                  cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
-    // same shared-memory carve-out for every kernel of the factorisation: no L1/shared reconfiguration
-    // between the back-to-back small launches of a panel
-    TGP_CUDA(cudaFuncSetAttribute(gemm_nt_sub_kernel<BN_, WARPS_M, WARPS_N, MIN_CTAS>,
-                                  cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  }
-  dim3 grid((unsigned)tgp_cdiv(Nc, BN_), (unsigned)tgp_cdiv(M, BM));
-  TGP_CHECK_ARG(grid.y <= 65535u, "M too large for one launch");
-  gemm_nt_sub_kernel<BN_, WARPS_M, WARPS_N, MIN_CTAS><<<grid, GEMM_THREADS, SMEM, st>>>(C, M, Nc, ldc, A, lda, B, ldb,
-                                                                                       Kd, lower_only);
-  TGP_LAUNCH_CHECK();
-  return TGP_OK;
-}
-
 static int gemm_nt_sub_launch(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
                               const double* B, int64_t ldb, int64_t Kd, int lower_only, cudaStream_t st) {
   if (M <= 0 || Nc <= 0 || Kd <= 0) return TGP_OK;
   TGP_CHECK_ARG((lda % 2 == 0) && (ldb % 2 == 0), "leading dimensions must be even (16-byte rows)");
   TGP_CHECK_ARG(((uintptr_t)A % 16 == 0) && ((uintptr_t)B % 16 == 0), "operands must be 16-byte aligned");
-  const int cfg = g_gemm_config >= 0 ? g_gemm_config : 1;
-  if (cfg == 0) return gemm_launch_cfg<128, 2, 4, 1>(C, M, Nc, ldc, A, lda, B, ldb, Kd, lower_only, st);
-  return gemm_launch_cfg<64, 4, 2, 2>(C, M, Nc, ldc, A, lda, B, ldb, Kd, lower_only, st);
+  constexpr int SMEM = STAGES * (BM + 64) * BK * 8;
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once)) {
+    TGP_CUDA(cudaFuncSetAttribute(gemm_nt_sub_kernel<64, 4, 2, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
+    // same shared-memory carve-out for every kernel of the factorisation: no L1/shared reconfiguration
+    // between the back-to-back small launches of a panel
+    TGP_CUDA(cudaFuncSetAttribute(gemm_nt_sub_kernel<64, 4, 2, 2>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+  }
+  dim3 grid((unsigned)tgp_cdiv(Nc, 64), (unsigned)tgp_cdiv(M, BM));
+  TGP_CHECK_ARG(grid.y <= 65535u, "M too large for one launch");
+  gemm_nt_sub_kernel<64, 4, 2, 2><<<grid, GEMM_THREADS, SMEM, st>>>(C, M, Nc, ldc, A, lda, B, ldb, Kd, lower_only);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
 }
 
 extern "C" int tgp_pairbin_set_block_sums(int on);
 extern "C" int tgp_pairbin_set_fast_paths(int bits);
 extern "C" int tgp_pairbin_set_record_cap(int n);
-extern "C" int tgp_trsv_set_cluster(int v);
 extern "C" int tgp_bootbin_set_paths(int bits);
 extern "C" int tgp_set_option(const char* name, int value) {
-  if (name && !strcmp(name, "trsv_cluster")) return tgp_trsv_set_cluster(value);
-  if (name && !strcmp(name, "gemm_config")) { g_gemm_config = value; return TGP_OK; }
-  if (name && !strcmp(name, "potrf_lookahead")) { g_lookahead = value; return TGP_OK; }
-  if (name && !strcmp(name, "potrf_fused")) { g_fused_panel = value; return TGP_OK; }
-  if (name && !strcmp(name, "potrf_env_lookahead")) { g_env_lookahead = value; return TGP_OK; }
   if (name && !strcmp(name, "pairbin_block_sums")) return tgp_pairbin_set_block_sums(value);
   if (name && !strcmp(name, "pairbin_fast_paths")) return tgp_pairbin_set_fast_paths(value);
   if (name && !strcmp(name, "pairbin_record_cap")) return tgp_pairbin_set_record_cap(value);
   if (name && !strcmp(name, "bootbin_paths")) return tgp_bootbin_set_paths(value);
-  if (name && !strcmp(name, "potrf_ob") && value >= 0 && value % 512 == 0) { g_ob_large = value; return TGP_OK; }
   tgp_set_error("tgp_set_option: unknown option");
   return TGP_ERR_INVALID;
 }
 
 // ============================================================================================
-// potf2: unblocked Cholesky of an n x n (n <= 64) diagonal block, one CTA.
+// potf2: unblocked Cholesky of an n x n (n <= 64) diagonal block by one CTA (CTA 0 of the fused panel step below).
 // ============================================================================================
 constexpr int NB = 64;           // inner block
 constexpr int NB_PITCH = NB + 1;
@@ -364,16 +340,6 @@ __device__ __forceinline__ void potf2_store(const double* __restrict__ S, double
   }
 }
 
-__global__ void __launch_bounds__(256)
-potf2_kernel(double* __restrict__ A, int n, int64_t ld, int32_t* __restrict__ info, int64_t global_off) {
-  __shared__ double S[NB * NB_PITCH];
-  __shared__ double rdiag[NB];   // 1 / L[j][j]
-  potf2_load(S, A, n, ld);
-  __syncthreads();
-  potf2_smem(S, rdiag, n, info, global_off);
-  potf2_store(S, A, n, ld);
-}
-
 // ============================================================================================
 // trsm panel: B (M x nb) <- B * L^-T for an nb x nb (nb <= 64) lower-triangular L.  Thread per row,
 // right-looking over columns so the FMAs of one step are independent.
@@ -481,7 +447,6 @@ static int trsm_panel_launch(const double* L, int nb, int64_t ldl, double* B, in
     TGP_CUDA(cudaFuncSetAttribute(trsm_panel_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_SMEM));
     TGP_CUDA(cudaFuncSetAttribute(trsm_panel_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     TGP_CUDA(cudaFuncSetAttribute(trsm_panel_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    TGP_CUDA(cudaFuncSetAttribute(potf2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   }
   const bool full = (nb == NB) && ((ldb & 1) == 0) && (((uintptr_t)B & 15) == 0);
   const unsigned grid = (unsigned)tgp_cdiv(M, TRSM_ROWS);
@@ -492,7 +457,7 @@ static int trsm_panel_launch(const double* L, int nb, int64_t ldl, double* B, in
 }
 
 // ============================================================================================
-// Fused panel step.  A w-wide (w <= OB = 512) panel = the w x w diagonal block D at `Akk` plus `below` rows
+// Fused panel step.  A w-wide (w <= TGP_OB = 512) panel = the w x w diagonal block D at `Akk` plus `below` rows
 // stored under it.  ONE launch per 64-wide block column j factorises D's diagonal block (j,j) and solves every
 // row block under it, instead of the potf2 / trsm_panel / K=64 gemm chain (3 launches per block column inside D
 // plus ~15 for the rows below).  Inside the panel the off-diagonal blocks are LEFT-looking and the diagonal
@@ -834,7 +799,7 @@ panel_left_kernel(double* __restrict__ Akk, int64_t ld, int w, int64_t below, in
 }
 
 
-// Factorise the w x w (w <= OB) diagonal block at Akk and solve the `below` rows under it (L21 = A21 L11^-T).
+// Factorise the w x w (w <= TGP_OB) diagonal block at Akk and solve the `below` rows under it (L21 = A21 L11^-T).
 static int panel_factor(double* Akk, int64_t w, int64_t ld, int64_t below, int32_t* info, int64_t goff,
                         cudaStream_t st) {
   static TgpPerDeviceOnce attr_once;
@@ -856,12 +821,12 @@ static int panel_factor(double* Akk, int64_t w, int64_t ld, int64_t below, int32
 }
 
 // ============================================================================================
-// Blocked drivers (two levels: OB-wide outer blocks whose updates run on DMMA with Kd = OB,
-// NB-wide inner blocks handled by the FP64-ALU kernels above).
+// Blocked drivers (two levels: TGP_OB-wide block columns whose updates run on DMMA with Kd = TGP_OB, NB-wide
+// inner blocks handled by the kernels above).  A dense factor is the envelope factor whose row ends
+// (tgp_envelope_ends) are n in every block column.
 // ============================================================================================
-constexpr int OB = 512;
 
-// B (M x n) <- B * L^-T for an n x n (n <= OB) lower-triangular L, by recursive halving of the columns:
+// B (M x n) <- B * L^-T for an n x n (n <= TGP_OB) lower-triangular L, by recursive halving of the columns:
 //   [B1 B2] <- [B1 L11^-T,  (B2 - B1 L21^T) L22^-T]
 // so the updates are GEMMs with K = n/2, n/4, ... (large K, each C column block touched once per level)
 // and only the 64-wide leaves run the FP64-ALU substitution kernel.
@@ -877,57 +842,45 @@ static int trsm_rows_halving(const double* L, int64_t n, int64_t ldl, double* B,
   return trsm_rows_halving(L + h * ldl + h, n - h, ldl, B + h, M, ldb, st);
 }
 
-// B (M x n) <- B * L^-T, L n x n lower.  bs = block size of this level (OB: right-looking over OB-wide
-// column blocks with DMMA updates of everything to the right; the OB-wide diagonal solves use halving).
-static int trsm_rows_rec(const double* L, int64_t n, int64_t ldl, double* B, int64_t M, int64_t ldb, int bs,
-                         cudaStream_t st) {
-  if (bs == NB) return trsm_rows_halving(L, n, ldl, B, M, ldb, st);
-  for (int64_t k = 0; k < n; k += bs) {
-    const int64_t w = (n - k < bs) ? (n - k) : bs;
-    const double* Lkk = L + k * ldl + k;
-    double* Bk = B + k;
-    int rc = trsm_rows_halving(Lkk, w, ldl, Bk, M, ldb, st);
+// B (M x n) <- B * L^-T, right-looking over TGP_OB-wide block columns: the unknowns [k, c1) of block column b are
+// solved by halving, then enter only the unknowns [c1, ends[b]) -- 2 M n bw flop instead of M n^2 for an envelope.
+static int trsm_rows_blocked(const double* L, int64_t n, int64_t ld, const std::vector<int64_t>& ends, double* B,
+                             int64_t M, int64_t ldb, cudaStream_t st) {
+  for (int64_t k = 0, b = 0; k < n; k += TGP_OB, ++b) {
+    const int64_t w = (n - k < TGP_OB) ? (n - k) : TGP_OB;
+    const int64_t c1 = k + w;
+    int rc = trsm_rows_halving(L + k * ld + k, w, ld, B + k, M, ldb, st);
     if (rc) return rc;
-    const int64_t rest = n - k - w;
-    if (rest > 0) {
-      // B[:, k+w:] -= B[:, k:k+w] * L[k+w:, k:k+w]^T
-      rc = gemm_nt_sub_launch(B + k + w, M, rest, ldb, Bk, ldb, L + (k + w) * ldl + k, ldl, w, 0, st);
-      if (rc) return rc;
-    }
+    rc = gemm_nt_sub_launch(B + c1, M, ends[b] - c1, ldb, B + k, ldb, L + c1 * ld + k, ld, w, 0, st);
+    if (rc) return rc;
   }
   return TGP_OK;
 }
 
-// `extra` rows stored below the n x n matrix (right-hand sides as ROWS) are carried through the panel solves and
-// trailing updates, so that on exit they hold Y L^-T (= L^-1 y per row): the forward substitution at DMMA speed.
-static int potrf_rec(double* A, int64_t n, int64_t ld, int bs, int32_t* info, int64_t goff, cudaStream_t st,
-                     int64_t extra = 0) {
-  if (g_fused_panel) bs = OB;   // the fused panel kernel handles everything below the OB level
-  for (int64_t k = 0; k < n; k += bs) {
-    const int64_t w = (n - k < bs) ? (n - k) : bs;
+// Per TGP_OB-wide block column b: the fused panel step factorises the diagonal block and solves the rows
+// [c1, ends[b]) inside the envelope, then one lower-triangular DMMA update applies them to the trailing matrix inside
+// the envelope.  The rows [ends[b], n) of block column b are neither read nor written (they keep whatever the K build
+// left there: entries below 1e-40 amp for an envelope).  `extra` right-hand-side rows stored below the matrix (rows
+// n .. n + extra - 1) end as Y L^-T (= L^-1 y per row): the forward substitution at DMMA speed.  Where the envelope
+// reaches n they are contiguous with its rows and ride inside the panel solve and the update; elsewhere they take
+// their own row solve and update.  (Empty updates launch nothing.)
+static int potrf_blocked(double* A, int64_t n, int64_t ld, const std::vector<int64_t>& ends, int64_t extra,
+                         int32_t* info, cudaStream_t st) {
+  for (int64_t k = 0, b = 0; k < n; k += TGP_OB, ++b) {
+    const int64_t w = (n - k < TGP_OB) ? (n - k) : TGP_OB;
+    const int64_t c1 = k + w, below = ends[b] - c1;
+    const int64_t ride = (ends[b] == n) ? extra : 0;
     double* Akk = A + k * ld + k;
-    const int64_t rest = n - k - w;
-    int rc;
-    if (g_fused_panel) {
-      rc = panel_factor(Akk, w, ld, rest + extra, info, goff + k, st);
+    double* Ark = A + c1 * ld + k;      // the rows of this block column inside the envelope (+ the riding rows)
+    int rc = panel_factor(Akk, w, ld, below + ride, info, k, st);
+    if (rc) return rc;
+    rc = gemm_nt_sub_launch(A + c1 * ld + c1, below + ride, below, ld, Ark, ld, Ark, ld, w, 1, st);
+    if (rc) return rc;
+    if (extra > ride) {
+      double* Aek = A + n * ld + k;
+      rc = trsm_rows_halving(Akk, w, ld, Aek, extra, ld, st);
       if (rc) return rc;
-    } else {
-      if (bs == NB) {
-        potf2_kernel<<<1, 256, 0, st>>>(Akk, (int)w, ld, info, goff + k);
-        TGP_LAUNCH_CHECK();
-        rc = TGP_OK;
-      } else {
-        rc = potrf_rec(Akk, w, ld, NB, info, goff + k, st);
-      }
-      if (rc) return rc;
-      if (rest + extra > 0) {
-        rc = trsm_rows_rec(Akk, w, ld, A + (k + w) * ld + k, rest + extra, ld, NB, st);
-        if (rc) return rc;
-      }
-    }
-    if (rest > 0) {
-      double* Ark = A + (k + w) * ld + k;  // rows below the diagonal block (+ the extra right-hand-side rows)
-      rc = gemm_nt_sub_launch(A + (k + w) * ld + (k + w), rest + extra, rest, ld, Ark, ld, Ark, ld, w, 1, st);
+      rc = gemm_nt_sub_launch(A + n * ld + c1, extra, below, ld, Aek, ld, Ark, ld, w, 0, st);
       if (rc) return rc;
     }
   }
@@ -935,15 +888,14 @@ static int potrf_rec(double* A, int64_t n, int64_t ld, int bs, int32_t* info, in
 }
 
 // --------------------------------------------------------------------------------------------
-// Look-ahead driver for large N.  The OB-wide panel (diagonal factorisation + solve of the rows
-// below) is a chain of ~40 small, latency-bound launches; run on its own high-priority stream it
-// hides under the previous step's big trailing update:
+// Look-ahead driver for large N.  The panel of an outer block (diagonal factorisation + solve of the rows below) is
+// a chain of small, latency-bound launches; run on its own high-priority stream it hides under the previous step's
+// big trailing update:
 //   panel stream P : panel(b) .. wait U2(b-1) .. U1(b) = update of the NEXT panel's column block only
 //   caller stream U: wait panel(b) .. U2(b) = update of everything right of the next panel
 // U1(b) and U2(b) write disjoint blocks; panel(b+1) needs U1(b) and U2(b-1) only, so U2(b) overlaps
 // with panel(b+1).  The caller's stream is joined with P before returning.
 // --------------------------------------------------------------------------------------------
-#include <vector>
 // Helper stream + events of the look-ahead schedule: one set per host thread AND device (streams and events
 // belong to the device that was current when they were created).
 struct LookaheadCtx {
@@ -972,7 +924,14 @@ static LookaheadCtx* lookahead_ctx() {
   }
   return &L;
 }
-static int potrf_lookahead(double* A, int64_t n, int64_t ld, int32_t* info, cudaStream_t U, int64_t extra = 0) {
+
+// Outer blocks of width obl (a multiple of TGP_OB), each factorised as TGP_OB-wide sub-panels solved against all rows
+// below them, with one K = TGP_OB update of the outer block's later columns in between.  The rows of an outer block
+// end at the envelope of its first TGP_OB block column, and the `extra` rows ride through every panel and update: so
+// an envelope runs with obl = TGP_OB and extra = 0, and only a dense factor (ends n everywhere) takes wider blocks or
+// extra rows.
+static int potrf_lookahead(double* A, int64_t n, int64_t ld, const std::vector<int64_t>& ends, int64_t extra,
+                           int64_t obl, int32_t* info, cudaStream_t U) {
   LookaheadCtx* Lp = lookahead_ctx();
   if (!Lp) {
     tgp_set_error("potrf: could not create the look-ahead stream: %s", cudaGetErrorString(cudaGetLastError()));
@@ -980,70 +939,46 @@ static int potrf_lookahead(double* A, int64_t n, int64_t ld, int32_t* info, cuda
   }
   LookaheadCtx& L = *Lp;
   cudaStream_t P = L.panel;
-  // K = 1024 trailing updates amortise the C read-modify-write better once the updates dominate (measured: K = 1024 from N ~ 14k, 2048 from ~ 28k)
-  const int64_t OBL = (g_ob_large > 0) ? g_ob_large : (n >= 28000 ? 2048 : (n >= 14000 ? 1024 : 512));
-  const int64_t nblk = tgp_cdiv(n, OBL);
-  if (!L.ensure((size_t)(3 + 2 * nblk))) {
+  const int64_t nblk = tgp_cdiv(n, obl);
+  if (!L.ensure((size_t)(2 + 2 * nblk))) {
     tgp_set_error("potrf: cudaEventCreate failed: %s", cudaGetErrorString(cudaGetLastError()));
     return TGP_ERR_CUDA;
   }
-  cudaEvent_t e_start = L.get(0);
-  TGP_CUDA(cudaEventRecord(e_start, U));
-  TGP_CUDA(cudaStreamWaitEvent(P, e_start, 0));
-  // event slots: 1 + 2*b = panel(b) done, 2 + 2*b = U2(b) done
+  TGP_CUDA(cudaEventRecord(L.get(0), U));
+  TGP_CUDA(cudaStreamWaitEvent(P, L.get(0), 0));
+  // event slots: 1 + 2 b = panel(b) done (on P), 2 + 2 b = U2(b) done (on U), 1 + 2 nblk = the join
   for (int64_t b = 0; b < nblk; ++b) {
-    const int64_t k = b * OBL;
-    const int64_t w = (n - k < OBL) ? (n - k) : OBL;
-    double* Akk = A + k * ld + k;
-    int rc = TGP_OK;
-    const int64_t rest = n - k - w;
-    if (g_fused_panel) {
-      // OB-wide sub-panels, each solved against ALL rows below it; the columns of the later sub-panels of this
-      // outer block are brought up to date by one K = OB update in between
-      for (int64_t s = 0; s < w; s += OB) {
-        const int64_t ws = (w - s < OB) ? (w - s) : OB;
-        double* Ass = A + (k + s) * ld + (k + s);
-        const int64_t below_s = (n - (k + s) - ws) + extra;
-        rc = panel_factor(Ass, ws, ld, below_s, info, k + s, P);
-        if (rc) return rc;
-        const int64_t rem = w - s - ws;
-        if (rem > 0) {
-          double* Aop = A + (k + s + ws) * ld + (k + s);
-          rc = gemm_nt_sub_launch(A + (k + s + ws) * ld + (k + s + ws), below_s, rem, ld, Aop, ld, Aop, ld, ws, 1, P);
-          if (rc) return rc;
-        }
-      }
-    } else {
-      rc = potrf_rec(Akk, w, ld, w > OB ? OB : NB, info, k, P);
+    const int64_t k = b * obl;
+    const int64_t w = (n - k < obl) ? (n - k) : obl;
+    const int64_t c1 = k + w, below = ends[k / TGP_OB] - c1;
+    int rc;
+    for (int64_t s = 0; s < w; s += TGP_OB) {
+      const int64_t ws = (w - s < TGP_OB) ? (w - s) : TGP_OB;
+      double* Ass = A + (k + s) * ld + (k + s);
+      const int64_t below_s = (c1 - (k + s) - ws) + below + extra;
+      rc = panel_factor(Ass, ws, ld, below_s, info, k + s, P);
       if (rc) return rc;
-      if (rest + extra > 0) {
-        double* Ark = A + (k + w) * ld + k;
-        rc = trsm_rows_rec(Akk, w, ld, Ark, rest + extra, ld, w > OB ? OB : NB, P);
-        if (rc) return rc;
-      }
+      double* Aop = A + (k + s + ws) * ld + (k + s);
+      rc = gemm_nt_sub_launch(A + (k + s + ws) * ld + (k + s + ws), below_s, w - s - ws, ld, Aop, ld, Aop, ld, ws, 1,
+                              P);
+      if (rc) return rc;
     }
-    cudaEvent_t e_panel = L.get(1 + 2 * b);
-    TGP_CUDA(cudaEventRecord(e_panel, P));
-    if (rest <= 0) {
-      TGP_CUDA(cudaStreamWaitEvent(U, e_panel, 0));
-      break;
-    }
-    double* Ark = A + (k + w) * ld + k;
-    const int64_t w2 = (rest < OBL) ? rest : OBL;
-    TGP_CUDA(cudaStreamWaitEvent(U, e_panel, 0));
+    TGP_CUDA(cudaEventRecord(L.get(1 + 2 * b), P));
+    TGP_CUDA(cudaStreamWaitEvent(U, L.get(1 + 2 * b), 0));
+    // everything the next panel reads must be final: the U2 updates up to block b-1 (stream order on U covers the
+    // earlier ones)
     if (b >= 1) TGP_CUDA(cudaStreamWaitEvent(P, L.get(2 + 2 * (b - 1)), 0));
-    // U1(b): next panel's column block, all rows below the current panel (+ extra rows)
-    rc = gemm_nt_sub_launch(A + (k + w) * ld + (k + w), rest + extra, w2, ld, Ark, ld, Ark, ld, w, 1, P);
+    double* Ark = A + c1 * ld + k;
+    const int64_t w2 = (below < obl) ? below : obl, rest2 = below - w2;
+    rc = gemm_nt_sub_launch(A + c1 * ld + c1, below + extra, w2, ld, Ark, ld, Ark, ld, w, 1, P);   // U1(b)
     if (rc) return rc;
-    // U2(b): everything to the right of the next panel
-    const int64_t rest2 = rest - w2;
-    if (rest2 > 0) {
-      rc = gemm_nt_sub_launch(A + (k + w + w2) * ld + (k + w + w2), rest2 + extra, rest2, ld, Ark + w2 * ld, ld,
-                              Ark + w2 * ld, ld, w, 1, U);
-      if (rc) return rc;
-    }
+    rc = gemm_nt_sub_launch(A + (c1 + w2) * ld + (c1 + w2), rest2 + extra, rest2, ld, Ark + w2 * ld, ld, Ark + w2 * ld,
+                            ld, w, 1, U);                                                            // U2(b)
+    if (rc) return rc;
     TGP_CUDA(cudaEventRecord(L.get(2 + 2 * b), U));
   }
+  TGP_CUDA(cudaEventRecord(L.get(1 + 2 * nblk), P));
+  TGP_CUDA(cudaStreamWaitEvent(U, L.get(1 + 2 * nblk), 0));
   return TGP_OK;
 }
 
@@ -1053,204 +988,61 @@ static int check_mat(const double* A, int64_t N, int64_t ld) {
   return 0;
 }
 
-static int potrf_with_rows(double* A, int64_t N, int64_t ld, int64_t extra, int32_t* info, cudaStream_t st) {
+// The look-ahead schedule from N = 3 TGP_OB, for a dense factor or an envelope factor without extra rows; the
+// sequential one otherwise.
+static int potrf_run(double* A, int64_t N, int64_t ld, const int64_t* row_end, int64_t extra, int32_t* info,
+                     cudaStream_t st) {
   TGP_CUDA(cudaMemsetAsync(info, 0, sizeof(int32_t), st));
   if (N == 0) return TGP_OK;
-  if (g_lookahead && N >= 3 * OB) return potrf_lookahead(A, N, ld, info, st, extra);
-  return potrf_rec(A, N, ld, N > OB ? OB : NB, info, 0, st, extra);
+  const std::vector<int64_t> ends = tgp_envelope_ends(row_end, N);
+  if (N >= 3 * TGP_OB && (!row_end || extra == 0)) {
+    // K = 1024 trailing updates amortise the C read-modify-write better once the updates dominate (measured: K = 1024
+    // from N ~ 14k, 2048 from ~ 28k)
+    const int64_t obl = row_end ? TGP_OB : (N >= 28000 ? 2048 : (N >= 14000 ? 1024 : TGP_OB));
+    return potrf_lookahead(A, N, ld, ends, extra, obl, info, st);
+  }
+  return potrf_blocked(A, N, ld, ends, extra, info, st);
 }
 
 extern "C" int tgp_potrf(double* A, int64_t N, int64_t ld, int32_t* info, void* stream) {
   TGP_CHECK_ARG(!check_mat(A, N, ld), "A must be 16-byte aligned with even ld >= N");
   TGP_CHECK_ARG(info != nullptr, "info");
-  return potrf_with_rows(A, N, ld, 0, info, (cudaStream_t)stream);
+  return potrf_run(A, N, ld, nullptr, 0, info, (cudaStream_t)stream);
 }
 
 extern "C" int tgp_potrf_rows(double* A, int64_t N, int64_t ld, int64_t nrows, int32_t* info, void* stream) {
   TGP_CHECK_ARG(!check_mat(A, N, ld), "A must be 16-byte aligned with even ld >= N");
   TGP_CHECK_ARG(info != nullptr && nrows >= 0, "info/nrows");
-  return potrf_with_rows(A, N, ld, nrows, info, (cudaStream_t)stream);
+  return potrf_run(A, N, ld, nullptr, nrows, info, (cudaStream_t)stream);
 }
 
 // --------------------------------------------------------------------------------------------
 // Envelope (variable-band) Cholesky.  With the points sorted along one axis, a kernel that is below 1e-40 of its
 // amplitude beyond a coordinate difference d_cut gives a matrix whose row i starts (to 1e-40) at the first point
-// within d_cut of point i; a Cholesky factor keeps the envelope of its matrix.  Per OB-wide block column b the caller
-// states row_end[b]: the rows [row_end[b], N) of that block column are (numerically) zero in K and therefore in L, so
-// the panel solve and the trailing update stop there: N bw^2 flop instead of N^3 / 3 for a band of bw rows.  Rows
-// outside the envelope are neither read nor written (they keep whatever the K build left there: entries below
-// 1e-40 amp).  `extra` right-hand-side rows below the matrix are carried through as in potrf_rec.
+// within d_cut of point i; a Cholesky factor keeps the envelope of its matrix.  Per TGP_OB-wide block column b the
+// caller states row_end[b]: the rows [row_end[b], N) of that block column are (numerically) zero in K and therefore in
+// L, so the panel solve and the trailing update stop there: N bw^2 flop instead of N^3 / 3 for a band of bw rows.
 // --------------------------------------------------------------------------------------------
-static int potrf_envelope(double* A, int64_t n, int64_t ld, const int64_t* row_end, int32_t* info, cudaStream_t st,
-                          int64_t extra) {
-  int64_t prev_end = 0;
-  for (int64_t k = 0, b = 0; k < n; k += OB, ++b) {
-    const int64_t w = (n - k < OB) ? (n - k) : OB;
-    const int64_t c1 = k + w;
-    int64_t re = row_end[b];
-    if (re < prev_end) re = prev_end;   // an envelope never shrinks from one block column to the next
-    if (re < c1) re = c1;
-    if (re > n) re = n;
-    prev_end = re;
-    const int64_t below = re - c1;
-    double* Akk = A + k * ld + k;
-    double* Ark = A + c1 * ld + k;      // the rows of this block column inside the envelope
-    double* Aek = A + n * ld + k;       // the extra rows
-    int rc;
-    if (g_fused_panel) {
-      rc = panel_factor(Akk, w, ld, below, info, k, st);
-      if (rc) return rc;
-    } else {
-      rc = potrf_rec(Akk, w, ld, NB, info, k, st);
-      if (rc) return rc;
-      if (below > 0) {
-        rc = trsm_rows_rec(Akk, w, ld, Ark, below, ld, NB, st);
-        if (rc) return rc;
-      }
-    }
-    if (extra > 0) {
-      rc = trsm_rows_rec(Akk, w, ld, Aek, extra, ld, NB, st);
-      if (rc) return rc;
-    }
-    if (below > 0) {
-      rc = gemm_nt_sub_launch(A + c1 * ld + c1, below, below, ld, Ark, ld, Ark, ld, w, 1, st);
-      if (rc) return rc;
-      if (extra > 0) {
-        rc = gemm_nt_sub_launch(A + n * ld + c1, extra, below, ld, Aek, ld, Ark, ld, w, 0, st);
-        if (rc) return rc;
-      }
-    }
-  }
-  return TGP_OK;
-}
-
-// The same factorisation on two streams, as potrf_lookahead does for the dense matrix: the panel of block column b+1
-// (a chain of 8 latency-bound launches) runs on the high-priority stream P while the caller's stream U still applies
-// block column b's update to everything right of that panel.
-//   P: panel(b) .. wait U2(b-1) .. U1(b) = update of the next panel's columns (rows inside the envelope) .. panel(b+1)
-//   U: wait panel(b) .. U2(b) = update of the columns right of the next panel
-// U1(b) and U2(b) write disjoint column ranges; U1(b+1) is ordered after U2(b) (both touch the columns right of panel
-// b+2's left edge).  No extra right-hand-side rows here (tgp_loglike_env uses the sweeps).
-static int potrf_envelope_lookahead(double* A, int64_t n, int64_t ld, const int64_t* row_end, int32_t* info,
-                                    cudaStream_t U) {
-  LookaheadCtx* Lp = lookahead_ctx();
-  if (!Lp) {
-    tgp_set_error("potrf_env: could not create the look-ahead stream: %s", cudaGetErrorString(cudaGetLastError()));
-    return TGP_ERR_CUDA;
-  }
-  LookaheadCtx& L = *Lp;
-  cudaStream_t P = L.panel;
-  const int64_t nblk = tgp_cdiv(n, (int64_t)OB);
-  if (!L.ensure((size_t)(4 + 2 * nblk))) {
-    tgp_set_error("potrf_env: cudaEventCreate failed: %s", cudaGetErrorString(cudaGetLastError()));
-    return TGP_ERR_CUDA;
-  }
-  TGP_CUDA(cudaEventRecord(L.get(0), U));
-  TGP_CUDA(cudaStreamWaitEvent(P, L.get(0), 0));
-  int64_t prev_end = 0;
-  // event slots: 1 + 2 b = panel(b) done (on P), 2 + 2 b = U2(b) done (on U)
-  for (int64_t b = 0; b < nblk; ++b) {
-    const int64_t k = b * OB;
-    const int64_t w = (n - k < OB) ? (n - k) : OB;
-    const int64_t c1 = k + w;
-    int64_t re = row_end[b];
-    if (re < prev_end) re = prev_end;
-    if (re < c1) re = c1;
-    if (re > n) re = n;
-    prev_end = re;
-    const int64_t below = re - c1;
-    double* Akk = A + k * ld + k;
-    double* Ark = A + c1 * ld + k;
-    int rc = panel_factor(Akk, w, ld, below, info, k, P);
-    if (rc) return rc;
-    cudaEvent_t e_panel = L.get(1 + 2 * b);
-    // U2(b) is released right after panel(b), beside U1(b).  Option value 2 releases it after U1(b) instead (U1 then
-    // has the SMs to itself and the next panel starts earlier): measured 33.1 ms against 31.8 ms at N = 40k -- the
-    // panel CTAs (134 KB of shared memory) cannot become resident beside U2's CTAs anyway, so a later U2 only ends later.
-    const bool u2_beside_u1 = (g_env_lookahead != 2);
-    if (u2_beside_u1) {
-      TGP_CUDA(cudaEventRecord(e_panel, P));
-      TGP_CUDA(cudaStreamWaitEvent(U, e_panel, 0));
-    }
-    // everything the next panel reads must be final: the U2 updates up to block b-1 (stream order on U covers the
-    // earlier ones)
-    if (b >= 1) TGP_CUDA(cudaStreamWaitEvent(P, L.get(2 + 2 * (b - 1)), 0));
-    if (below > 0) {
-      const int64_t w2 = (below < OB) ? below : OB;
-      rc = gemm_nt_sub_launch(A + c1 * ld + c1, below, w2, ld, Ark, ld, Ark, ld, w, 1, P);            // U1(b)
-      if (rc) return rc;
-    }
-    if (!u2_beside_u1) {
-      TGP_CUDA(cudaEventRecord(e_panel, P));
-      TGP_CUDA(cudaStreamWaitEvent(U, e_panel, 0));
-    }
-    if (below > 0) {
-      const int64_t w2 = (below < OB) ? below : OB;
-      const int64_t rest2 = below - w2;
-      if (rest2 > 0) {
-        rc = gemm_nt_sub_launch(A + (c1 + w2) * ld + (c1 + w2), rest2, rest2, ld, Ark + w2 * ld, ld, Ark + w2 * ld,
-                                ld, w, 1, U);                                                         // U2(b)
-        if (rc) return rc;
-      }
-    }
-    TGP_CUDA(cudaEventRecord(L.get(2 + 2 * b), U));
-  }
-  // join: the caller's stream continues after the last panel-stream work
-  TGP_CUDA(cudaEventRecord(L.get(3 + 2 * nblk), P));
-  TGP_CUDA(cudaStreamWaitEvent(U, L.get(3 + 2 * nblk), 0));
-  return TGP_OK;
-}
-
-static int check_envelope(const int64_t* row_end, int64_t nblocks, int64_t N) {
-  return row_end == nullptr || nblocks != tgp_cdiv(N, (int64_t)OB);
-}
-
-extern "C" int tgp_envelope_block(void) { return OB; }
+extern "C" int tgp_envelope_block(void) { return TGP_OB; }
 
 extern "C" int tgp_potrf_env(double* A, int64_t N, int64_t ld, const int64_t* row_end, int64_t nblocks,
                              int64_t nrows, int32_t* info, void* stream) {
   TGP_CHECK_ARG(!check_mat(A, N, ld), "A must be 16-byte aligned with even ld >= N");
   TGP_CHECK_ARG(info != nullptr && nrows >= 0, "info/nrows");
-  TGP_CHECK_ARG(!check_envelope(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
-  cudaStream_t st = (cudaStream_t)stream;
-  TGP_CUDA(cudaMemsetAsync(info, 0, sizeof(int32_t), st));
-  if (N == 0) return TGP_OK;
-  if (g_env_lookahead && g_fused_panel && nrows == 0 && N >= 3 * OB)
-    return potrf_envelope_lookahead(A, N, ld, row_end, info, st);
-  return potrf_envelope(A, N, ld, row_end, info, st, nrows);
-}
-
-// B <- B L^-T for a factor with the envelope row_end: after the block of unknowns [k, c1) is solved it only enters
-// the unknowns [c1, row_end[b]) -- 2 M N bw flop instead of M N^2.
-static int trsm_rows_envelope(const double* L, int64_t n, int64_t ld, const int64_t* row_end, double* B, int64_t M,
-                              int64_t ldb, cudaStream_t st) {
-  int64_t prev_end = 0;
-  for (int64_t k = 0, b = 0; k < n; k += OB, ++b) {
-    const int64_t w = (n - k < OB) ? (n - k) : OB;
-    const int64_t c1 = k + w;
-    int64_t re = row_end[b];
-    if (re < prev_end) re = prev_end;
-    if (re < c1) re = c1;
-    if (re > n) re = n;
-    prev_end = re;
-    int rc = trsm_rows_rec(L + k * ld + k, w, ld, B + k, M, ldb, NB, st);
-    if (rc) return rc;
-    if (re > c1) {
-      rc = gemm_nt_sub_launch(B + c1, M, re - c1, ldb, B + k, ldb, L + c1 * ld + k, ld, w, 0, st);
-      if (rc) return rc;
-    }
-  }
-  return TGP_OK;
+  TGP_CHECK_ARG(row_end && tgp_envelope_ok(row_end, nblocks, N),
+                "row_end must hold one entry per tgp_envelope_block() columns");
+  return potrf_run(A, N, ld, row_end, nrows, info, (cudaStream_t)stream);
 }
 
 extern "C" int tgp_trsm_rows_env(const double* L, int64_t N, int64_t ld, const int64_t* row_end, int64_t nblocks,
                                  double* B, int64_t M, int64_t ldb, void* stream) {
   TGP_CHECK_ARG(!check_mat(L, N, ld), "L must be 16-byte aligned with even ld >= N");
   TGP_CHECK_ARG(M >= 0 && ldb >= N, "M/ldb");
-  TGP_CHECK_ARG(!check_envelope(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(row_end && tgp_envelope_ok(row_end, nblocks, N),
+                "row_end must hold one entry per tgp_envelope_block() columns");
   if (M == 0 || N == 0) return TGP_OK;
   TGP_CHECK_ARG(B && (ldb % 2 == 0) && ((uintptr_t)B % 16 == 0), "B must be 16-byte aligned with even ldb");
-  return trsm_rows_envelope(L, N, ld, row_end, B, M, ldb, (cudaStream_t)stream);
+  return trsm_rows_blocked(L, N, ld, tgp_envelope_ends(row_end, N), B, M, ldb, (cudaStream_t)stream);
 }
 
 extern "C" int tgp_trsm_rows(const double* L, int64_t N, int64_t ld, double* B, int64_t M, int64_t ldb,
@@ -1259,7 +1051,7 @@ extern "C" int tgp_trsm_rows(const double* L, int64_t N, int64_t ld, double* B, 
   TGP_CHECK_ARG(M >= 0 && ldb >= N, "M/ldb");
   if (M == 0 || N == 0) return TGP_OK;
   TGP_CHECK_ARG(B && (ldb % 2 == 0) && ((uintptr_t)B % 16 == 0), "B must be 16-byte aligned with even ldb");
-  return trsm_rows_rec(L, N, ld, B, M, ldb, N > OB ? OB : NB, (cudaStream_t)stream);
+  return trsm_rows_blocked(L, N, ld, tgp_envelope_ends(nullptr, N), B, M, ldb, (cudaStream_t)stream);
 }
 
 extern "C" int tgp_gemm_nt_sub(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
@@ -1387,8 +1179,7 @@ sumsq_kernel(const double* __restrict__ w, int64_t N, double* __restrict__ out1)
 static int loglike_args(const double* X, const double* y, int64_t N, const double* work, const double* alpha,
                         const double* out, const int32_t* info, const int64_t* row_end, int64_t nblocks) {
   TGP_CHECK_ARG(N > 0 && X && y && work && alpha && out && info, "null pointer / N");
-  TGP_CHECK_ARG(row_end == nullptr || !check_envelope(row_end, nblocks, N),
-                "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(tgp_envelope_ok(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
   return TGP_OK;
 }
 
@@ -1565,11 +1356,11 @@ extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, co
 }
 
 // ============================================================================================
-// Batches of independent problems (tgp_loglike_batch).  The schedule of potrf_rec with y riding along as row N, run
-// once over the panel steps of the largest problem: every launch covers each problem that still has columns at that
-// step (CTAs of the others exit), and each CTA runs the body of the single-problem kernel on its problem's block.
-// For N >= 3 OB the single call takes the look-ahead driver, whose U1 / U2 updates split the same K = OB update by
-// columns: per element the same DMMA chain, so the factor is the same bit for bit.
+// Batches of independent problems (tgp_loglike_batch).  The schedule of potrf_blocked with y riding along as row N,
+// run once over the panel steps of the largest problem: every launch covers each problem that still has columns at
+// that step (CTAs of the others exit), and each CTA runs the body of the single-problem kernel on its problem's block.
+// For N >= 3 TGP_OB the single call takes the look-ahead driver, whose U1 / U2 updates split the same K = TGP_OB update
+// by columns: per element the same DMMA chain, so the factor is the same bit for bit.
 // ============================================================================================
 // grid: (problem, CTA of the panel launch); the CTAs 0 of all problems are dispatched before any CTA that waits.
 __global__ void __launch_bounds__(PL_THREADS, 2)
@@ -1578,7 +1369,7 @@ panel_left_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int j, i
   const int b = blockIdx.x;
   const int64_t N = pr[b].N;
   if (k >= N) return;
-  const int w = (int)(N - k < OB ? N - k : OB);
+  const int w = (int)(N - k < TGP_OB ? N - k : TGP_OB);
   const int ndiag = (w + NB - 1) / NB;
   if (j >= ndiag) return;
   const int64_t below = N - k - w + 1;
@@ -1593,7 +1384,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 2)
 gemm_trail_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int tiles_n) {
   const int b = blockIdx.x;
   const int64_t N = pr[b].N;
-  const int64_t w = N - k < OB ? N - k : OB, rest = N - k - w;
+  const int64_t w = N - k < TGP_OB ? N - k : TGP_OB, rest = N - k - w;
   if (rest <= 0) return;
   const int64_t m0 = (int64_t)(blockIdx.y / tiles_n) * BM, n0 = (int64_t)(blockIdx.y % tiles_n) * 64;
   if (m0 >= rest + 1 || n0 >= rest) return;
@@ -1618,13 +1409,13 @@ int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, i
   int64_t nmax = 0;
   for (int32_t b = 0; b < B; ++b) nmax = Nh[b] > nmax ? Nh[b] : nmax;
   unsigned epoch = 0;   // the flags start at 0 and every panel launch of this call takes the next epoch
-  for (int64_t k = 0; k < nmax; k += OB) {
-    const int64_t wmax = nmax - k < OB ? nmax - k : OB;
+  for (int64_t k = 0; k < nmax; k += TGP_OB) {
+    const int64_t wmax = nmax - k < TGP_OB ? nmax - k : TGP_OB;
     for (int j = 0; j < (int)tgp_cdiv(wmax, NB); ++j) {
       int64_t ctas = 0;   // the largest launch of a problem at this step
       for (int32_t b = 0; b < B; ++b) {
         if (Nh[b] <= k) continue;
-        const int64_t w = Nh[b] - k < OB ? Nh[b] - k : OB, ndiag = tgp_cdiv(w, NB);
+        const int64_t w = Nh[b] - k < TGP_OB ? Nh[b] - k : TGP_OB, ndiag = tgp_cdiv(w, NB);
         if (j >= ndiag) continue;
         const int64_t c = (ndiag - j) + tgp_cdiv(Nh[b] - k - w + 1, NB);
         ctas = c > ctas ? c : ctas;

@@ -16,7 +16,6 @@
 // over the lower triangle inside the envelope: with w_ij = alpha_i alpha_j - Z_ij and K_ij = a f(q_ij),
 //   d logL / d ln a = 1/2 sum_ij w_ij a f(q_ij),   d logL / d m_uv = 1/2 sum_ij w_ij a f'(q_ij) d q_ij / d m_uv.
 #include <string.h>
-#include <vector>
 #include "tgp_common.cuh"
 #include "profile_dq.cuh"
 #include "profile_policy.cuh"
@@ -30,7 +29,6 @@ extern "C" int tgp_loglike(const double* X, const double* y, const double* yerr2
 extern "C" int tgp_loglike_env(const double* X, const double* y, const double* yerr2, int64_t N, const tgp_kernel* k,
                                double* work, int64_t ld, double* alpha, int want_alpha, double* out, int32_t* info,
                                const int64_t* row_end, int64_t nblocks, void* stream);
-extern "C" int tgp_envelope_block(void);
 extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N,
                                const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
                                double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream);
@@ -38,7 +36,6 @@ extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, co
                                  const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
                                  double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream);
 
-constexpr int SB = 512;            // block columns of the recurrence: the envelope's block (tgp_envelope_block)
 constexpr int GT = 64;             // contraction tile edge
 constexpr int GT_THREADS = 256;
 
@@ -51,9 +48,9 @@ static int64_t grad_tiles(int64_t N) {
 // ncols partial sums per contraction tile: 4 for one term, 4 nterms + 1 for a sum
 static int64_t grad_work_doubles(int64_t N, int ncols) {
   if (N < 1) N = 1;
-  const int64_t selinv = 2 * (int64_t)SB * SB + (int64_t)SB * even64(N);   // -W^T, W^T, T^T
+  const int64_t selinv = 2 * (int64_t)TGP_OB * TGP_OB + (int64_t)TGP_OB * even64(N);   // -W^T, W^T, T^T
   const int64_t partials = ncols * grad_tiles(N);                           // contraction partial sums
-  return (selinv > partials ? selinv : partials) + even64(tgp_cdiv(N, SB));  // + the device copy of row_end
+  return (selinv > partials ? selinv : partials) + even64(tgp_cdiv(N, TGP_OB));  // + the device copy of row_end
 }
 
 extern "C" int64_t tgp_selinv_work_doubles(int64_t N) { return grad_work_doubles(N, 4); }
@@ -123,49 +120,30 @@ static int mirror_launch(const double* src, double* dst, int64_t rows, int64_t c
 static int check_args_mat(const double* A, int64_t N, int64_t ld) {
   return N <= 0 || ld < N || !A || (ld & 1) || ((uintptr_t)A & 15);
 }
-static int check_env(const int64_t* row_end, int64_t nblocks, int64_t N) {
-  return row_end != nullptr && nblocks != tgp_cdiv(N, (int64_t)SB);
-}
-
-// Row ends as the factorisation uses them: clamped to [end of the block, N] and made non-decreasing.
-static std::vector<int64_t> clamped_row_end(const int64_t* row_end, int64_t N) {
-  const int64_t nb = tgp_cdiv(N, (int64_t)SB);
-  std::vector<int64_t> re((size_t)nb);
-  int64_t prev = 0;
-  for (int64_t b = 0; b < nb; ++b) {
-    const int64_t c1 = (b + 1) * SB < N ? (b + 1) * SB : N;
-    int64_t r = row_end ? row_end[b] : N;
-    if (r < prev) r = prev;
-    if (r < c1) r = c1;
-    if (r > N) r = N;
-    re[(size_t)b] = prev = r;
-  }
-  return re;
-}
 
 static int selinv_run(double* A, int64_t N, int64_t ld, const std::vector<int64_t>& re, double* scratch,
                       cudaStream_t st) {
   void* sv = (void*)st;
-  double* NWT = scratch;                  // -W^T, SB x SB
-  double* WT = scratch + SB * SB;         //  W^T, SB x SB
-  double* TT = scratch + 2 * SB * SB;     //  T^T, SB x ldt
+  double* NWT = scratch;                          // -W^T, TGP_OB x TGP_OB
+  double* WT = scratch + TGP_OB * TGP_OB;         //  W^T, TGP_OB x TGP_OB
+  double* TT = scratch + 2 * TGP_OB * TGP_OB;     //  T^T, TGP_OB x ldt
   const int64_t ldt = even64(N);
   const unsigned eg = 2 * (unsigned)tgp_num_sms();
   for (int64_t b = (int64_t)re.size() - 1; b >= 0; --b) {
-    const int64_t k = b * SB, w = (N - k < SB) ? (N - k) : SB, c1 = k + w, m = re[(size_t)b] - c1;
+    const int64_t k = b * TGP_OB, w = (N - k < TGP_OB) ? (N - k) : TGP_OB, c1 = k + w, m = re[(size_t)b] - c1;
     double* Akk = A + k * ld + k;
     double* L21 = A + c1 * ld + k;        // becomes Z[R, J]
     double* ZJR = A + k * ld + c1;        // upper-triangle storage of Z[J, R]
     int rc;
-    neg_identity_kernel<<<eg, 256, 0, st>>>(NWT, (int)w, SB);
+    neg_identity_kernel<<<eg, 256, 0, st>>>(NWT, (int)w, TGP_OB);
     TGP_LAUNCH_CHECK();
-    rc = tgp_trsm_rows(Akk, w, ld, NWT, w, SB, sv);            // rows of -I times L11^-T: -W^T
+    rc = tgp_trsm_rows(Akk, w, ld, NWT, w, TGP_OB, sv);        // rows of -I times L11^-T: -W^T
     if (rc) return rc;
-    negate_kernel<<<eg, 256, 0, st>>>(NWT, WT, (int)w, SB);
+    negate_kernel<<<eg, 256, 0, st>>>(NWT, WT, (int)w, TGP_OB);
     TGP_LAUNCH_CHECK();
     if (m > 0) {
       TGP_CUDA(cudaMemset2DAsync(TT, ldt * sizeof(double), 0, m * sizeof(double), w, st));
-      rc = tgp_gemm_nt_sub(TT, w, m, ldt, NWT, SB, L21, ld, w, 0, sv);              // T^T = W^T L21^T
+      rc = tgp_gemm_nt_sub(TT, w, m, ldt, NWT, TGP_OB, L21, ld, w, 0, sv);          // T^T = W^T L21^T
       if (rc) return rc;
       TGP_CUDA(cudaMemset2DAsync(L21, ld * sizeof(double), 0, w * sizeof(double), m, st));
       rc = tgp_gemm_nt_sub(L21, m, w, ld, A + c1 * ld + c1, ld, TT, ldt, m, 0, sv);  // Z[R, J] = -Z[R, R] T
@@ -174,7 +152,7 @@ static int selinv_run(double* A, int64_t N, int64_t ld, const std::vector<int64_
       if (rc) return rc;
     }
     TGP_CUDA(cudaMemset2DAsync(Akk, ld * sizeof(double), 0, w * sizeof(double), w, st));
-    rc = tgp_gemm_nt_sub(Akk, w, w, ld, NWT, SB, WT, SB, w, 1, sv);                 // + W^T W
+    rc = tgp_gemm_nt_sub(Akk, w, w, ld, NWT, TGP_OB, WT, TGP_OB, w, 1, sv);         // + W^T W
     if (rc) return rc;
     if (m > 0) {
       rc = tgp_gemm_nt_sub(Akk, w, w, ld, TT, ldt, ZJR, ld, m, 1, sv);               // - T^T Z[R, J]
@@ -189,10 +167,10 @@ static int selinv_run(double* A, int64_t N, int64_t ld, const std::vector<int64_
 extern "C" int tgp_selinv(double* L, int64_t N, int64_t ld, const int64_t* row_end, int64_t nblocks, double* scratch,
                           void* stream) {
   TGP_CHECK_ARG(!check_args_mat(L, N, ld), "L must be 16-byte aligned with even ld >= N > 0");
-  TGP_CHECK_ARG(!check_env(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(tgp_envelope_ok(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
   TGP_CHECK_ARG(scratch && ((uintptr_t)scratch & 15) == 0,
                 "scratch: 16-byte aligned buffer of tgp_selinv_work_doubles(N) doubles");
-  return selinv_run(L, N, ld, clamped_row_end(row_end, N), scratch, (cudaStream_t)stream);
+  return selinv_run(L, N, ld, tgp_envelope_ends(row_end, N), scratch, (cudaStream_t)stream);
 }
 
 // ---- gradient contraction ---------------------------------------------------------------------------------------
@@ -228,7 +206,7 @@ grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const doub
   while ((I + 1) * (I + 2) / 2 <= t) ++I;
   const int64_t J = t - I * (I + 1) / 2;
   const int64_t r0 = I * GT, c0 = J * GT;
-  const int64_t rend = re_dev ? re_dev[c0 / SB] : N;   // one past the last envelope row of this block column
+  const int64_t rend = re_dev ? re_dev[c0 / TGP_OB] : N;   // one past the last envelope row of this block column
   const int tid = threadIdx.x;
   if (r0 >= rend) {
     if (tid < 4) partials[prof.partial(t, tid)] = 0.0;
@@ -367,7 +345,7 @@ static int grad_args(const double* X, const double* y, int64_t N, double* work, 
                      const double* scratch) {
   TGP_CHECK_ARG(N > 0 && X && y && alpha && out && info, "null pointer / N");
   TGP_CHECK_ARG(!check_args_mat(work, N, ld), "work must be 16-byte aligned with even ld >= N");
-  TGP_CHECK_ARG(!check_env(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
+  TGP_CHECK_ARG(tgp_envelope_ok(row_end, nblocks, N), "row_end must hold one entry per tgp_envelope_block() columns");
   TGP_CHECK_ARG(scratch && ((uintptr_t)scratch & 15) == 0,
                 "scratch: 16-byte aligned buffer of tgp_selinv_work_doubles(N) doubles");
   TGP_CHECK_ARG(grad_tiles(N) < (1ll << 31), "matrix too large for one launch");
@@ -381,7 +359,7 @@ static int grad_tail(const double* X, int64_t N, const P& prof, int nterms, int 
                      const double* alpha, double* out, const int32_t* info, const int64_t* row_end, double* scratch,
                      cudaStream_t st, int nrhs = 1) {
   const int64_t ntiles = grad_tiles(N);
-  const std::vector<int64_t> re = clamped_row_end(row_end, N);
+  const std::vector<int64_t> re = tgp_envelope_ends(row_end, N);
   int rc = selinv_run(work, N, ld, re, scratch, st);
   if (rc) return rc;
   // the selected-inverse scratch is free again: tile partials at the front, the envelope at the back

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <vector>
 #include "../../include/treegp_b200.h"
 #include "vk_profile.cuh"
 
@@ -36,6 +37,32 @@ void tgp_set_error(const char* fmt, ...);
   } while (0)
 
 static inline int64_t tgp_cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
+
+// ---- envelopes ------------------------------------------------------------------------------
+// The blocked Cholesky works on TGP_OB-wide block columns, and an envelope (variable-band factor) gives one row end per
+// block column: tgp_envelope_block().
+constexpr int TGP_OB = 512;
+
+// row_end holds one entry per block column (NULL: no envelope, for the callers that allow it)
+static inline bool tgp_envelope_ok(const int64_t* row_end, int64_t nblocks, int64_t N) {
+  return row_end == nullptr || nblocks == tgp_cdiv(N, TGP_OB);
+}
+
+// Row ends as the factorisation uses them: clamped to [end of the block, N] and made non-decreasing (an envelope never
+// shrinks from one block column to the next); N in every block column without row_end.
+static inline std::vector<int64_t> tgp_envelope_ends(const int64_t* row_end, int64_t N) {
+  std::vector<int64_t> ends((size_t)tgp_cdiv(N, TGP_OB));
+  int64_t prev = 0;
+  for (size_t b = 0; b < ends.size(); ++b) {
+    const int64_t c1 = ((int64_t)b + 1) * TGP_OB < N ? ((int64_t)b + 1) * TGP_OB : N;
+    int64_t r = row_end ? row_end[b] : N;
+    if (r < prev) r = prev;
+    if (r < c1) r = c1;
+    if (r > N) r = N;
+    ends[b] = prev = r;
+  }
+  return ends;
+}
 
 int tgp_num_sms();
 

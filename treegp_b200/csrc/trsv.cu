@@ -780,8 +780,7 @@ static size_t trsv_smem_bytes(bool fwd, int slabs_per_cta, int R = 1) {
          (size_t)slabs_per_cta * TS * 8 * (fwd ? 1 : 8) * R;
 }
 
-static int g_trsv_cluster = -1;   // option "trsv_cluster": -1 automatic, 1 no clusters, 2 / 4 / 8 cluster size
-extern "C" int tgp_trsv_set_cluster(int v) { g_trsv_cluster = v; return TGP_OK; }
+static bool g_clusters_refused = false;   // set when a cooperative launch with clusters is refused: none from then on
 
 // CTAs of one cooperative launch: as many as are co-resident (one per SM: the kernel takes most of the shared
 // memory), in clusters of CS when a cluster size is in use.
@@ -823,14 +822,11 @@ static void trsv_config(const TrsvParams& P, int& cs, int& G) {
   cs = 1;
   G = P.G;
   const size_t smem1 = trsv_smem_bytes(FWD, (P.nb + P.G - 1) / P.G);
-  if (g_trsv_cluster != 1 && P.nb >= 4) {
-    const int tries[3] = {8, 4, 2};
-    for (int t = 0; t < 3; ++t) {
-      const int c2 = tries[t];
-      if (g_trsv_cluster > 1 && c2 != g_trsv_cluster) continue;
+  if (!g_clusters_refused && P.nb >= 4) {
+    for (const int c2 : {8, 4, 2}) {
       if (P.nb < c2) continue;
       const int g = trsv_grid<FWD, 1>(P.nb, c2, smem1 + 4096);
-      if (g >= c2 && (g_trsv_cluster > 1 || 10 * g >= 9 * (P.nb < P.G ? (P.nb / c2) * c2 : P.G))) {
+      if (g >= c2 && 10 * g >= 9 * (P.nb < P.G ? (P.nb / c2) * c2 : P.G)) {
         cs = c2;
         G = g;
         break;
@@ -868,7 +864,7 @@ static int trsv_launch(const TrsvParams& P0, cudaStream_t st) {
   cudaError_t e = cudaLaunchKernelEx(&cfg, trsv_sweep_kernel<FWD, R>, P);
   if (e != cudaSuccess && cs > 1) {                // clusters + cooperative launch refused: go on without clusters
     cudaGetLastError();
-    g_trsv_cluster = 1;
+    g_clusters_refused = true;
     return trsv_launch<FWD, R>(P0, st);
   }
   TGP_CUDA(e);
