@@ -341,8 +341,9 @@ typedef enum {
  *                   below).  NULL: no block forms (TwoD: pair by pair; Log: the boxes are recomputed on the fly);
  *                   the counts are the same.
  * TwoD with work first books the pairs of super-chunks (256 consecutive points) that sit in one bin or vary along
- * one axis only, then runs in rounds of this rank's items: a classification pass books the other blocks that sit
- * in one bin and records the rest, then a second kernel processes the recorded blocks.  A round holds at most
+ * one axis only, and decides the 32-point blocks of the super pairs that span at most 2 x 2 bins (the range edge
+ * counting as one) in one more kernel.  Then it runs in rounds of this rank's items: a classification pass books the
+ * other blocks that sit in one bin and records the rest, then a second kernel processes the recorded blocks.  A round holds at most
  * 2^26 records (1 GiB of `work` at N >= ~4e5; fewer for smaller catalogues), about 8 rounds at N = 1e6. */
 int tgp_pairbin(const double* px, const double* py, const double* pk, const double* pw,
                 const int64_t* cat_off, int32_t ncat, int64_t max_cat_len, int32_t bin_type,
@@ -352,8 +353,9 @@ int tgp_pairbin(const double* px, const double* py, const double* pk, const doub
 
 /* Size (in doubles) of the optional scratch buffer of tgp_pairbin for catalogues of `total_points` points in
  * all (an upper bound on max_cat_len is enough): the chunk records of the pre-pass, the super-chunk records
- * (boxes, sums and sorted copies of 256-point super-chunks, about 48 MB at N = 1e6) and the block records of one
- * round, capped at 2^26 records of 16 bytes. */
+ * (boxes, sums and sorted copies of 256-point super-chunks, about 48 MB at N = 1e6), a list with room for every
+ * pair of super-chunks (16 bytes each: S (S - 1) / 2 entries for S = total_points / 256, about 122 MB at N = 1e6)
+ * and the block records of one round, capped at 2^26 records of 16 bytes. */
 int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat);
 
 /* Hilbert-curve keys of 2-D points on a 2^order x 2^order grid over the square
@@ -474,6 +476,11 @@ int tgp_pairbin_tile(void);
  * super-chunk pair in one bin, booked whole, [6] (TwoD) super-chunk pair with one varying axis, one rank query per row
  * point on the super-chunk's sorted copy.  The slots are disjoint.  Synchronous. */
 int tgp_pairbin_stats(unsigned long long* host8 /*host*/, int reset);
+
+/* Diagnostics: how many super-chunk pairs of all TwoD tgp_pairbin launches since the last reset spanned at most two
+ * bins per axis (the range edge counting as one) and had their 32-point blocks decided by the leaf kernel without
+ * block records.  Their blocks are tallied in the slots of tgp_pairbin_stats as usual.  Synchronous. */
+int tgp_pairbin_super_leaves(unsigned long long* host1 /*host*/, int reset);
 
 /* Test and measurement switches of the pair counts (tgp_pairbin_*, tgp_bootbin_twod), not needed for normal use.
  * Any other name is rejected with TGP_ERR_INVALID ("unknown option").

@@ -1,6 +1,6 @@
 """Two builds of the library compared on the bench.py 2PCF workload: one JSON file in --outdir (pairbin_split_probe.json).
 
-For each build (--lib, one or more paths; the first is the reference) and each of --rounds rounds, the builds
+For each build (--lib, one or more library files or source trees with their own build; the first is the reference) and each of --rounds rounds, the builds
 alternated, a fresh subprocess with TREEGP_B200_LIB pointing at the build times one TwoD count (CUDA events around
 backend.pairbin_packed, L2 overwritten before each, median of 3 after a warm-up) on the bench.py catalogue:
   n1m       N = 1e6, default max_sep (half the field diagonal), unweighted -- the bench value;
@@ -86,6 +86,8 @@ def worker(profile):
 
         count(c1, c1[5])
         backend.pairbin_stats(reset=True)
+        if hasattr(backend, "pairbin_super_leaves"):
+            backend.pairbin_super_leaves(reset=True)
         torch.cuda.synchronize()
         with tprofile(activities=[ProfilerActivity.CUDA]) as prof:
             count(c1, c1[5])
@@ -96,6 +98,8 @@ def worker(profile):
                 kern[ev.key] = {"ms": ev.device_time_total / 1e3, "launches": ev.count}
         out["kernels"] = kern
         st = backend.pairbin_stats(reset=True)
+        if hasattr(backend, "pairbin_super_leaves"):
+            out["super_pairs_leaf_kernel"] = backend.pairbin_super_leaves(reset=True)
         tot = sum(st.values())
         out["path_fractions"] = {k: v / tot for k, v in st.items()} if tot else st
     print("RESULT " + json.dumps(out), flush=True)
@@ -115,9 +119,16 @@ def main():
     libs = [os.path.abspath(p) for p in args.lib]
 
     def run(lib, profile=False):
-        env = dict(os.environ, TREEGP_B200_LIB=lib)
-        cmd = [sys.executable, os.path.abspath(__file__), "--worker"] + (["--profile"] if profile else [])
-        p = subprocess.run(cmd, env=env, capture_output=True, text=True, cwd=ROOT)
+        # a library file runs under this tree's binding; a directory is a whole tree (binding, library and this
+        # probe of its own), for builds whose C ABI differs from this one's
+        tree = lib if os.path.isdir(lib) else ROOT
+        env = dict(os.environ)
+        env.pop("TREEGP_B200_LIB", None)
+        if tree == ROOT:
+            env["TREEGP_B200_LIB"] = lib
+        cmd = [sys.executable, os.path.join(tree, "tools", "pairbin_split_probe.py"), "--worker"] + \
+            (["--profile"] if profile else [])
+        p = subprocess.run(cmd, env=env, capture_output=True, text=True, cwd=tree)
         for line in p.stdout.splitlines():
             if line.startswith("RESULT "):
                 return json.loads(line[7:])

@@ -106,6 +106,7 @@ SIGNATURES = {
     "tgp_vcorr": [_vp, _vp, _vp, _vp, _i64, _vp, _i32, _vp, _vp, _vp, _i32, _vp, _vp],
     "tgp_pairbin_tile": [],
     "tgp_pairbin_stats": [_vp, ctypes.c_int],
+    "tgp_pairbin_super_leaves": [_vp, ctypes.c_int],
     "tgp_set_option": [ctypes.c_char_p, ctypes.c_int],
     "tgp_microbench_fp64": [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)],
 }

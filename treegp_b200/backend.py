@@ -712,8 +712,9 @@ _PB_SCRATCH = {}
 
 
 def _pairbin_scratch(dev, doubles):
-    """The workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6, plus the block records of
-    one round of the two-pass TwoD count, at most 1 GiB), kept per
+    """The workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6, the super-chunk records and
+    the list of super pairs for the leaf kernel, ~170 MB, plus the block records of one round of the two-pass TwoD
+    count, at most 1 GiB), kept per
     (device, stream) and grown on demand: launches on one stream are ordered, so they can share it; launches on
     different streams get different buffers."""
     key = (dev.index, torch.cuda.current_stream(dev).cuda_stream)
@@ -869,6 +870,14 @@ def pairbin_stats(reset=True):
     keys = ("closed_form", "one_axis", "pairwise", "one_axis_sorted", "two_axis_sorted", "super_closed_form",
             "super_one_axis")
     return {k: int(buf[i]) for i, k in enumerate(keys)}
+
+
+def pairbin_super_leaves(reset=True):
+    """Super-chunk pairs decided by the TwoD leaf kernel since the last reset (see tgp_pairbin_super_leaves); kept
+    apart from pairbin_stats, whose values are pair counts that add up to the total."""
+    v = ctypes.c_ulonglong(0)
+    check(_cabi.load().tgp_pairbin_super_leaves(ctypes.byref(v), int(bool(reset))), "tgp_pairbin_super_leaves")
+    return int(v.value)
 
 
 def set_option(name, value):

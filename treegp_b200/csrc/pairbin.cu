@@ -27,8 +27,10 @@
 // runs the paths below over the recorded blocks only.  The classification needs none of the per-row register state
 // of the residual paths, so it runs at more warps per SM and the residual kernel's warm code no longer contains it.
 // Before the rounds, pairbin_super_kernel books the pairs of super-chunks (PB_SUPER chunks) that are out of range, sit
-// in one bin, or vary along one axis only (one rank query per row point on the super-chunk's sorted copy); the
-// classification pass skips their blocks and descends to the 32-point blocks only for the other super pairs.
+// in one bin, or vary along one axis only (one rank query per row point on the super-chunk's sorted copy), and lists
+// those that span at most 2 x 2 bins; pairbin_super_leaves_kernel decides the 32-point blocks of the listed pairs in
+// one launch, without records.  The classification pass skips the blocks of all of them and descends to the 32-point
+// blocks only for the other super pairs.
 //
 // Two instantiations per bin type (template parameter BS):
 //   BS = false  the pair-by-pair kernel: every pair of every in-range block is evaluated individually
@@ -110,6 +112,7 @@ struct PBParams {
   int4* recs;
   int* rec_cnt;
   unsigned long long* counter_next;
+  unsigned long long* slist_len;   // super kernel / leaf kernel: length of the TWO_AXIS super pair list (pb_super_list)
 };
 
 // Which path the pairs of all launches since the last reset took (in pairs): [0] closed form (block in one bin; TwoD:
@@ -1421,9 +1424,14 @@ __device__ __forceinline__ const double* pb_super_records(const PBParams& P) {
 //   CLOSED    every pair in range, in ONE forward bin per axis, and the mirrored window is its mirror image;
 //   ONE_AXIS  every pair in range, one such bin on one axis, exactly two forward bins [v0, v0 + 1] on the other whose
 //             mirrored window is the mirror image [nbins-2-v0, nbins-1-v0]; vx: x is the varying axis;
+//   TWO_AXIS  neither of the above, but every pair passes r2 >= lo2 and each axis spans at most two "bins", where the
+//             out-of-range region |d| >= max_sep counts as one, and its in-range mirrored window is the mirror image of
+//             the forward one (the range test is the same for both entries: fl(x_i - x_j) = -fl(x_j - x_i)).  x0, y0 =
+//             origin of the fixed 2 x 2 forward window [x0, x0 + 1] x [y0, y0 + 1] that holds every in-range pair;
 //   DESCEND   anything else, the diagonal (R == C) and short super-chunks: the chunks are classified one by one.
-// The super kernel books the first three; the classification pass skips every block of such a pair.
-enum { PB_S_OUT = 0, PB_S_CLOSED = 1, PB_S_ONE_AXIS = 2, PB_S_DESCEND = 3 };
+// The super kernel books CLOSED and ONE_AXIS and lists TWO_AXIS for the leaf kernel; the classification pass skips
+// every block of a super pair that is not DESCEND.
+enum { PB_S_OUT = 0, PB_S_CLOSED = 1, PB_S_ONE_AXIS = 2, PB_S_DESCEND = 3, PB_S_TWO_AXIS = 4 };
 __device__ __forceinline__ int pb_super_status(const double* __restrict__ srec, int64_t nsf, int64_t R, int64_t C,
                                                double M, double lo2, int nbins, const double* __restrict__ ed,
                                                int& x0, int& y0, bool& vx) {
@@ -1432,19 +1440,40 @@ __device__ __forceinline__ int pb_super_status(const double* __restrict__ srec, 
   const double4 b = *reinterpret_cast<const double4*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)C);
   int w[4];
   const int cls = pb_classify_twod<true>(a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, M, lo2, nbins, ed, w);
-  if (cls == PB_OUT) return PB_S_OUT;
-  if (cls != PB_REG_FULL) return PB_S_DESCEND;
+  if (cls == PB_OUT || cls == PB_GENERIC) return cls == PB_OUT ? PB_S_OUT : PB_S_DESCEND;
   x0 = w[0] & 0xffff;
   y0 = w[1] & 0xffff;
   const int rx0 = w[2] & 0xffff, ry0 = w[3] & 0xffff;
-  const bool one_x = (w[0] >> 16) == 0 && (w[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
-  const bool one_y = (w[1] >> 16) == 0 && (w[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
-  const bool clean_x = (w[0] >> 16) == 1 && (w[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
-  const bool clean_y = (w[1] >> 16) == 1 && (w[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
-  vx = one_y;
-  if (one_x && one_y) return PB_S_CLOSED;
-  if ((one_y && clean_x) || (one_x && clean_y)) return PB_S_ONE_AXIS;
-  return PB_S_DESCEND;
+  const int ex = w[0] >> 16, ey = w[1] >> 16;
+  if (cls == PB_REG_FULL) {
+    const bool one_x = ex == 0 && (w[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
+    const bool one_y = ey == 0 && (w[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
+    const bool clean_x = ex == 1 && (w[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
+    const bool clean_y = ey == 1 && (w[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
+    vx = one_y;
+    if (one_x && one_y) return PB_S_CLOSED;
+    if ((one_y && clean_x) || (one_x && clean_y)) return PB_S_ONE_AXIS;
+  }
+  if (nbins < 2) return PB_S_DESCEND;
+  // in-range windows [x0, x0 + ex] (mirrored: the mirror image) plus the out-of-range ends, at most two slots per axis
+  const double dx0 = b.x - a.y, dx1 = b.y - a.x, dy0 = b.z - a.w, dy1 = b.w - a.z;
+  const double nx = dx0 > 0.0 ? dx0 : (dx1 < 0.0 ? -dx1 : 0.0), ny = dy0 > 0.0 ? dy0 : (dy1 < 0.0 ? -dy1 : 0.0);
+  const bool mirror_x = (w[2] >> 16) == ex && rx0 == nbins - 1 - x0 - ex;
+  const bool mirror_y = (w[3] >> 16) == ey && ry0 == nbins - 1 - y0 - ey;
+  const int sx = ex + 1 + (dx1 >= M ? 1 : 0) + (dx0 <= -M ? 1 : 0);
+  const int sy = ey + 1 + (dy1 >= M ? 1 : 0) + (dy0 <= -M ? 1 : 0);
+  if (!mirror_x || !mirror_y || sx > 2 || sy > 2 || __dadd_rn(__dmul_rn(nx, nx), __dmul_rn(ny, ny)) < lo2)
+    return PB_S_DESCEND;
+  x0 = min(x0, nbins - 2);   // one in-range bin (nbins - 1 when the upper range edge is the other slot): either bit
+  y0 = min(y0, nbins - 2);
+  return PB_S_TWO_AXIS;
+}
+
+// The list of TWO_AXIS super pairs follows the super records: {length, work counter of the leaf kernel} at `work` words
+// 3 and 4, entries {cat, R, C, x0 | y0 << 16} here, room for every super pair of every catalogue.
+__device__ __forceinline__ int4* pb_super_list(const PBParams& P) {
+  return reinterpret_cast<int4*>(const_cast<double*>(pb_super_records(P)) +
+                                 (size_t)PB_SUPER_STRIDE * (size_t)(P.cat_off[P.ncat] / PB_SUPER_PTS + P.ncat + 2));
 }
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_CLASSIFY_MIN_CTAS)
@@ -1536,8 +1565,8 @@ pairbin_classify_kernel(PBParams P) {
       const double2 rsum = *reinterpret_cast<const double2*>(rec0 + (size_t)PB_STRIDE * (size_t)it.ib + 4);
       const int nlive = (it.ib == nblk - 1) ? tail : PB_CHUNK;
       int4* out = P.recs + (size_t)(q - P.q_begin) * (size_t)P.run;
-      // the super kernel books every super pair that is not DESCEND (on one rank); its blocks are skipped here on every
-      // rank.  Lane l decides super column cw + l; the chunks of the DESCEND ones are then classified 32 at a time.
+      // the super kernel books or lists every super pair that is not DESCEND (on one rank); its blocks are skipped here
+      // on every rank.  Lane l decides super column cw + l; the chunks of the DESCEND ones are then classified 32 at a time.
       const double* srec = pb_super_records(P) + (size_t)PB_SUPER_STRIDE * (size_t)(it.off / PB_SUPER_PTS + it.cat);
       const int64_t nsf = P.block_sums == 2 ? it.n / PB_SUPER_PTS : 0, sR = it.ib / PB_SUPER;
       for (int64_t cw = it.c_lo / PB_SUPER; cw * PB_SUPER < it.c_hi; cw += 32) {
@@ -1745,6 +1774,7 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
 //             predicate (monotone in c_j).  The upper bin gets n_C - pos pairs and k_i w_i x suffix(pos), the lower bin
 //             the rest.  The exact mirrored bits differ from the mirror image only for the columns between pos and
 //             pos_m = #{j : fl(c_j - c_i) <= -t_m}, nearly always none; those pairs are moved in global memory.
+//   TWO_AXIS  appended to the list of the leaf kernel (pairbin_super_leaves_kernel).
 // The warp histograms hold forward entries; the mirror image is added when they are written out.
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, 2)
@@ -1796,6 +1826,7 @@ pairbin_super_kernel(PBParams P) {
 
   const double M = P.hi, lo2 = P.lo2;
   const double* sup0 = pb_super_records(P);
+  int4* slist = pb_super_list(P);
   const int64_t nruns = (P.items_per_cat + 31) / 32;   // items_per_cat: super-chunks of the longest catalogue
   unsigned st_closed = 0, st_one = 0;   // super pairs
   int cur_cat = -1, since_flush = 0;
@@ -1824,6 +1855,14 @@ pairbin_super_kernel(PBParams P) {
     int x0 = 0, y0 = 0;
     bool vx = false;
     const int st = C > R ? pb_super_status(srec, nsf, R, C, M, lo2, nbins, ed, x0, y0, vx) : PB_S_DESCEND;
+    const unsigned two = __ballot_sync(0xffffffffu, st == PB_S_TWO_AXIS);
+    if (two) {   // appended for the leaf kernel: one atomic per warp step
+      unsigned long long base = 0;
+      if (lane == 0) base = atomicAdd(P.slist_len, (unsigned long long)__popc(two));
+      base = __shfl_sync(0xffffffffu, base, 0);
+      if (st == PB_S_TWO_AXIS)
+        slist[base + __popc(two & ((1u << lane) - 1u))] = make_int4(cat, (int)R, (int)C, x0 | (y0 << 16));
+    }
     if (st == PB_S_CLOSED) {
       const double2 csum = *reinterpret_cast<const double2*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)C + 4);
       const int o = y0 * nbins + x0;
@@ -1927,6 +1966,339 @@ pairbin_super_kernel(PBParams P) {
   if (st_one) atomicAdd(&g_pb_stats[6], (unsigned long long)PB_SUPER_PTS * PB_SUPER_PTS * st_one);
 }
 
+// Super pairs taken by the leaf kernel since the last reset (tgp_pairbin_super_leaves).  Diagnostics.
+__device__ unsigned long long g_pb_super_leaves;
+
+// Rank query with the bin predicate on the displacement itself: pos = #{j : fl(c_j - ci) < t} in a chunk's ascending
+// copy xs (4-ary search as pb_rank_query_g: 3 + 3 + 2 probes in three dependent steps).  fl(c_j - ci) is monotone in
+// c_j, so the bisection is exact.  Returns whether the exact mirrored bits agree: columns below pos need
+// fl(c_j - ci) <= tm (mirrored upper bit), columns from pos on need it false; only the neighbours of pos can fail.
+__device__ __forceinline__ bool pb_rank_query_d(const double* __restrict__ xs, double ci, double t, double tm,
+                                                int& pos) {
+  const int b = 8 * ((xs[7] - ci < t ? 1 : 0) + (xs[15] - ci < t ? 1 : 0) + (xs[23] - ci < t ? 1 : 0));
+  const int sp = b + 2 * ((xs[b + 1] - ci < t ? 1 : 0) + (xs[b + 3] - ci < t ? 1 : 0) + (xs[b + 5] - ci < t ? 1 : 0));
+  pos = sp + (xs[sp] - ci < t ? 1 : 0) + (xs[sp + 1] - ci < t ? 1 : 0);
+  return (pos == 0 || xs[pos - 1] - ci <= tm) && (pos == PB_CHUNK || !(xs[pos] - ci <= tm));
+}
+
+// Leaf classes inside a TWO_AXIS super pair (pairbin_super_leaves_kernel)
+enum { PB_L_OUT = 0, PB_L_CLOSED = 1, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD = 4, PB_L_PAIRS = 5, PB_L_EDGE = 6 };
+
+// The leaf kernel: the TWO_AXIS super pairs of the list, one per warp step (persistent CTAs, device-side counter; the
+// length is read on the device).  A super pair's window [x0, x0 + 1] x [y0, y0 + 1] holds every in-range pair and its
+// mirrored window is the mirror image, so the lanes keep four forward bins in registers for the whole super pair
+// (sums over all pairs, over the x-bit, the y-bit and both bits; inclusion-exclusion at the end).  Its 64 leaf blocks
+// (32 x 32 points) are decided as pass B decides them, from pb_classify_twod on the chunk boxes of the pre-pass:
+//   closed    in ONE bin whose mirrored window is its mirror image: booked by the classifying lane (2 blocks per lane)
+//             from the chunk sums, no point loaded;
+//   one axis  one rank query per row point on the chunk's copy sorted along the varying axis;
+//   2 x 2     (both windows clean) the column-bit and row-bit sums from two rank queries, the "both bits" quadrant
+//             pair by pair;
+//   otherwise pair by pair over the staged chunk, with the range test where the range edge runs through the block.
+// A failed mirrored-bit check at the split hands the block to the pair-by-pair loop, which counts the pairs whose
+// exact mirrored bin is not the mirror image and moves them in global memory afterwards (as pass B's fix_mirror).
+// The bit predicates compare the displacement fl(c_j - c_i) with the bin thresholds directly (no per-lane coordinate
+// thresholds).  The warp histograms hold forward entries; the mirror image is added when they are written out.
+#ifndef PB_LEAVES_MIN_CTAS
+#define PB_LEAVES_MIN_CTAS 2
+#endif
+template <bool WEIGHTED>
+__global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_LEAVES_MIN_CTAS)
+pairbin_super_leaves_kernel(PBParams P) {
+  extern __shared__ __align__(16) unsigned char pb_smem[];
+  const int nb = P.nb, nbins = P.nbins;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  double* ed = reinterpret_cast<double*>(pb_smem);                          // nbins + 1 (padded to even)
+  double2* cxy_all = reinterpret_cast<double2*>(ed + ((nbins + 2) & ~1));   // [warps][32]
+  double* ck_all = reinterpret_cast<double*>(cxy_all + P.warps * PB_CHUNK);  // [warps][32]
+  double* cw_all = ck_all + P.warps * PB_CHUNK;                              // [warps][32]
+  double* hs_all = cw_all + P.warps * PB_CHUNK;                              // [warps][nb]  sum wk wk
+  double* hw_all = hs_all + (size_t)P.warps * nb;                            // [warps][nb]  sum w w     (WEIGHTED)
+  unsigned* hc_all = reinterpret_cast<unsigned*>(hw_all + (WEIGHTED ? (size_t)P.warps * nb : 0));
+  double2* cxy = cxy_all + warp * PB_CHUNK;
+  double* ck = ck_all + warp * PB_CHUNK;
+  double* cw = cw_all + warp * PB_CHUNK;
+  double* my_s = hs_all + (size_t)warp * nb;
+  double* my_w = hw_all + (size_t)warp * nb;
+  unsigned* my_c = hc_all + (size_t)warp * nb;
+  for (int i = tid; i <= nbins; i += blockDim.x) ed[i] = P.edges[i];
+  for (int i = lane; i < nb; i += 32) {
+    my_s[i] = 0.0;
+    my_c[i] = 0u;
+    if constexpr (WEIGHTED) my_w[i] = 0.0;
+  }
+  __syncthreads();
+
+  auto flush_hist = [&](int cat) {   // forward entries of bin b + those of its mirror image, then clear
+    __syncwarp();
+    if (cat >= 0) {
+      for (int b = lane; b < nb; b += 32) {
+        const int bm = nb - 1 - b;
+        const unsigned long long c = (unsigned long long)my_c[b] + (unsigned long long)my_c[bm];
+        if (c) {
+          const size_t o = (size_t)cat * nb + b;
+          atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + o, c);
+          atomicAdd(P.sumwkk + o, my_s[b] + my_s[bm]);
+          atomicAdd(P.sumw + o, WEIGHTED ? my_w[b] + my_w[bm] : (double)c);
+        }
+      }
+      __syncwarp();
+      for (int b = lane; b < nb; b += 32) {
+        my_c[b] = 0u;
+        my_s[b] = 0.0;
+        if constexpr (WEIGHTED) my_w[b] = 0.0;
+      }
+    }
+    __syncwarp();
+  };
+
+  const double M = P.hi, lo2 = P.lo2;
+  const int4* slist = pb_super_list(P);
+  const unsigned long long nlist = *P.slist_len;
+  unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0;   // leaf blocks, super pairs
+  int cur_cat = -1, since_flush = 0;
+  while (true) {
+    unsigned long long q = 0;
+    if (lane == 0) q = atomicAdd(P.counter, 1ull);
+    q = __shfl_sync(0xffffffffu, q, 0);
+    if (q >= nlist) break;
+    const int4 e = slist[q];
+    const int cat = e.x, wx0 = e.w & 0xffff, wy0 = e.w >> 16;
+    // <= 2^16 pairs per super pair and 2^31 / 2^16 super pairs per flush keep the 32-bit warp histogram counts exact
+    if (cat != cur_cat || since_flush >= (1 << 14)) {
+      flush_hist(cur_cat);
+      cur_cat = cat;
+      since_flush = 0;
+    }
+    ++since_flush;
+    ++st_pairs;
+    const int64_t off = P.cat_off[cat];
+    const int64_t r0 = (int64_t)e.y * PB_SUPER, c0 = (int64_t)e.z * PB_SUPER;   // first row / column chunk
+    const double* rec0 = P.boxes + (size_t)PB_STRIDE * (size_t)(off / PB_CHUNK + cat);
+    // bits of the window: forward upper bin dx >= tx; the mirrored entry's upper bin -dx >= ed[nbins-1-x0] <=> dx <= mx
+    const double tx = ed[wx0 + 1], ty = ed[wy0 + 1], mx = -ed[nbins - 1 - wx0], my = -ed[nbins - 1 - wy0];
+    // the four forward bins of the super pair, per lane: all pairs, x-bit, y-bit, both bits
+    unsigned n_t = 0u, n_x = 0u, n_y = 0u, n_xy = 0u;
+    double s_t = 0.0, s_x = 0.0, s_y = 0.0, s_xy = 0.0, w_t = 0.0, w_x = 0.0, w_y = 0.0, w_xy = 0.0;
+
+    // ---- classify the 64 leaf blocks: lane l takes column chunk l % 8 against row chunks l / 8 and l / 8 + 4 ----
+    const double* crec = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + (lane & 7));
+    const double4 cb = *reinterpret_cast<const double4*>(crec);
+    const double2 cs = *reinterpret_cast<const double2*>(crec + 4);
+    int code[2];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const double* rrec = rec0 + (size_t)PB_STRIDE * (size_t)(r0 + (lane >> 3) + 4 * h);
+      const double4 rb = *reinterpret_cast<const double4*>(rrec);
+      int win[4];
+      const int cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, cb.x, cb.y, cb.z, cb.w, M, lo2, nbins, ed, win);
+      const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
+      const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
+      const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
+      const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
+      const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
+      const int bx = x0 - wx0, by = y0 - wy0;   // window bits of an axis in one bin
+      int c = PB_L_OUT;
+      if (cls == PB_REG_CHECK) c = PB_L_EDGE;
+      else if (cls == PB_REG_FULL) {
+        if (one_x && one_y) {
+          const double2 rs = *reinterpret_cast<const double2*>(rrec + 4);
+          const double s = rs.x * cs.x, w = WEIGHTED ? rs.y * cs.y : 0.0;
+          const unsigned n = (unsigned)(PB_CHUNK * PB_CHUNK);
+          n_t += n; s_t += s; w_t += w;
+          if (bx) { n_x += n; s_x += s; w_x += w; }
+          if (by) { n_y += n; s_y += s; w_y += w; }
+          if (bx && by) { n_xy += n; s_xy += s; w_xy += w; }
+          ++st_closed;
+        } else if (one_y) c = PB_L_ONE_X | (by << 3);      // x varies, the y bit is constant
+        else if (one_x) c = PB_L_ONE_Y | (bx << 3);
+        else c = (clean_x && clean_y && (P.fast_paths & 2)) ? PB_L_QUAD : PB_L_PAIRS;
+      }
+      code[h] = c;
+    }
+    const unsigned act0 = __ballot_sync(0xffffffffu, code[0] != PB_L_OUT);
+    const unsigned act1 = __ballot_sync(0xffffffffu, code[1] != PB_L_OUT);
+
+    // ---- the other leaf blocks, one row chunk at a time: lane = row point ----
+    int staged = -1;   // column chunk staged in cxy / ck / cw
+    auto stage = [&](int c) {
+      if (c == staged) return;
+      const int64_t j = off + (c0 + c) * PB_CHUNK + lane;
+      double wj = 1.0;
+      if constexpr (WEIGHTED) wj = P.pw[j];
+      __syncwarp();
+      cxy[lane] = make_double2(P.px[j], P.py[j]);
+      ck[lane] = P.pk[j] * wj;
+      if constexpr (WEIGHTED) cw[lane] = wj;
+      __syncwarp();
+      staged = c;
+    };
+#pragma unroll 1
+    for (int rk = 0; rk < PB_SUPER; ++rk) {
+      unsigned m = ((rk < 4 ? act0 : act1) >> ((rk & 3) * 8)) & 0xffu;
+      if (!m) continue;
+      const int codes = rk < 4 ? code[0] : code[1];
+      const int64_t i = off + (r0 + rk) * PB_CHUNK + lane;
+      const double xi = P.px[i], yi = P.py[i];
+      double wi = 1.0;
+      if constexpr (WEIGHTED) wi = P.pw[i];
+      const double ki = P.pk[i] * wi;
+      // a block's column sums of k_j w_j (w_j) over all pairs, the x-bit, the y-bit and both bits, times this row
+      // point's k_i w_i (w_i)
+      auto book = [&](double at, double ax, double ay, double axy, double bt, double bx, double by, double bxy) {
+        s_t = fma(ki, at, s_t); s_x = fma(ki, ax, s_x); s_y = fma(ki, ay, s_y); s_xy = fma(ki, axy, s_xy);
+        if constexpr (WEIGHTED) {
+          w_t = fma(wi, bt, w_t); w_x = fma(wi, bx, w_x); w_y = fma(wi, by, w_y); w_xy = fma(wi, bxy, w_xy);
+        }
+      };
+      while (m) {
+        const int c = __ffs(m) - 1;
+        m &= m - 1;
+        const int lc = __shfl_sync(0xffffffffu, codes, (rk & 3) * 8 + c);
+        const int cls = lc & 7, cbit = lc >> 3;
+        const double csk = __shfl_sync(0xffffffffu, cs.x, c);
+        double csw = 0.0;
+        if constexpr (WEIGHTED) csw = __shfl_sync(0xffffffffu, cs.y, c);
+        const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + c) + PB_SLOT;   // sorted copies of the chunk
+        bool per_pair = cls >= PB_L_PAIRS;
+        if (cls == PB_L_ONE_X || cls == PB_L_ONE_Y) {
+          const bool vx = cls == PB_L_ONE_X;
+          const double* xs = vx ? srt : srt + 3 * PB_CHUNK;
+          int pos;
+          const bool ok = pb_rank_query_d(xs, vx ? xi : yi, vx ? tx : ty, vx ? mx : my, pos);
+          if (__all_sync(0xffffffffu, ok)) {
+            const unsigned bc = (unsigned)(PB_CHUNK - pos);
+            const double bs = pos < PB_CHUNK ? xs[PB_CHUNK + pos] : 0.0;
+            double bw = 0.0;
+            if constexpr (WEIGHTED) bw = pos < PB_CHUNK ? xs[2 * PB_CHUNK + pos] : 0.0;
+            // the varying axis' bit: the rank query; the constant axis' bit: cbit for every pair
+            const unsigned cc = cbit ? (unsigned)PB_CHUNK : 0u;
+            const double ck_ = cbit ? csk : 0.0, cw_ = cbit ? csw : 0.0;
+            n_t += PB_CHUNK;
+            n_x += vx ? bc : cc;
+            n_y += vx ? cc : bc;
+            n_xy += cbit ? bc : 0u;
+            book(csk, vx ? bs : ck_, vx ? ck_ : bs, cbit ? bs : 0.0, csw, vx ? bw : cw_, vx ? cw_ : bw, cbit ? bw : 0.0);
+            ++st_sorted;
+            continue;
+          }
+          ++st_1d;   // (rare) a column within rounding of a bin edge: pair by pair
+          per_pair = true;
+        } else if (cls == PB_L_QUAD) {
+          stage(c);
+          double qs = 0.0, qw = 0.0;
+          unsigned qc = 0u;
+#pragma unroll 4
+          for (int jj = 0; jj < PB_CHUNK; ++jj) {
+            const double2 pj = cxy[jj];
+            const bool p = (pj.x - xi >= tx) && (pj.y - yi >= ty);
+            const double mk = p ? 1.0 : 0.0;
+            qs = fma(ck[jj], mk, qs);
+            if constexpr (WEIGHTED) qw = fma(cw[jj], mk, qw);
+            qc += p ? 1u : 0u;
+          }
+          int posx, posy;
+          const bool okx = pb_rank_query_d(srt, xi, tx, mx, posx);
+          const bool oky = pb_rank_query_d(srt + 3 * PB_CHUNK, yi, ty, my, posy);
+          if (__all_sync(0xffffffffu, okx && oky)) {
+            n_t += PB_CHUNK;
+            n_x += (unsigned)(PB_CHUNK - posx);
+            n_y += (unsigned)(PB_CHUNK - posy);
+            n_xy += qc;
+            double bx = 0.0, by = 0.0;
+            if constexpr (WEIGHTED) {
+              bx = posx < PB_CHUNK ? srt[2 * PB_CHUNK + posx] : 0.0;
+              by = posy < PB_CHUNK ? srt[5 * PB_CHUNK + posy] : 0.0;
+            }
+            book(csk, posx < PB_CHUNK ? srt[PB_CHUNK + posx] : 0.0, posy < PB_CHUNK ? srt[4 * PB_CHUNK + posy] : 0.0, qs,
+                 csw, bx, by, qw);
+            ++st_quad;
+            continue;
+          }
+          per_pair = true;
+        }
+        if (!per_pair) continue;
+        // pair by pair over the raw points of the chunk: every in-range pair sits in the window; EDGE blocks test the
+        // range per pair (r2 >= lo2 holds for every pair of a TWO_AXIS super pair)
+        if (cls != PB_L_ONE_X && cls != PB_L_ONE_Y) ++st_pw;
+        stage(c);
+        const bool check = cls == PB_L_EDGE;
+        unsigned mmc = 0u;
+        double a_t = 0.0, a_x = 0.0, a_y = 0.0, a_xy = 0.0, b_t = 0.0, b_x = 0.0, b_y = 0.0, b_xy = 0.0;
+#pragma unroll 2
+        for (int jj = 0; jj < PB_CHUNK; ++jj) {
+          const double2 pj = cxy[jj];
+          const double dx = pj.x - xi, dy = pj.y - yi;
+          if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
+          const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
+          const double kj = ck[jj];
+          double wj = 0.0;
+          if constexpr (WEIGHTED) wj = cw[jj];
+          const double fx = px ? 1.0 : 0.0, fy = py ? 1.0 : 0.0, fxy = (px && py) ? 1.0 : 0.0;
+          n_t += 1u; n_x += px ? 1u : 0u; n_y += py ? 1u : 0u; n_xy += (px && py) ? 1u : 0u;
+          a_t += kj; a_x = fma(kj, fx, a_x); a_y = fma(kj, fy, a_y); a_xy = fma(kj, fxy, a_xy);
+          if constexpr (WEIGHTED) { b_t += wj; b_x = fma(wj, fx, b_x); b_y = fma(wj, fy, b_y); b_xy = fma(wj, fxy, b_xy); }
+          mmc += ((px != qx) && (py != qy)) ? 0u : 1u;
+        }
+        book(a_t, a_x, a_y, a_xy, b_t, b_x, b_y, b_xy);
+        if (__any_sync(0xffffffffu, mmc != 0u) && mmc) {
+          // (rare) pairs whose exact mirrored bin is not the mirror image of the forward bin: -1 at the assumed bin,
+          // +1 at the exact one, directly in global memory
+          const size_t g = (size_t)cat * nb;
+          for (int jj = 0; jj < PB_CHUNK; ++jj) {
+            const double2 pj = cxy[jj];
+            const double dx = pj.x - xi, dy = pj.y - yi;
+            if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
+            const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
+            if ((px != qx) && (py != qy)) continue;
+            const int assumed = (nbins - 1 - (wy0 + (py ? 1 : 0))) * nbins + (nbins - 1 - (wx0 + (px ? 1 : 0)));
+            const int exact = (nbins - 2 - wy0 + (qy ? 1 : 0)) * nbins + (nbins - 2 - wx0 + (qx ? 1 : 0));
+            const double kk = ki * ck[jj];
+            double ww = 1.0;
+            if constexpr (WEIGHTED) ww = wi * cw[jj];
+            atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + assumed, ~0ull);   // -1 (mod 2^64)
+            atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + exact, 1ull);
+            atomicAdd(P.sumwkk + g + assumed, -kk);
+            atomicAdd(P.sumwkk + g + exact, kk);
+            atomicAdd(P.sumw + g + assumed, -ww);
+            atomicAdd(P.sumw + g + exact, ww);
+          }
+        }
+      }
+    }
+
+    // ---- the four bins of the window into the warp histogram (forward entries) ----
+    n_t = warp_sum_u(n_t); n_x = warp_sum_u(n_x); n_y = warp_sum_u(n_y); n_xy = warp_sum_u(n_xy);
+    s_t = warp_sum(s_t); s_x = warp_sum(s_x); s_y = warp_sum(s_y); s_xy = warp_sum(s_xy);
+    if constexpr (WEIGHTED) { w_t = warp_sum(w_t); w_x = warp_sum(w_x); w_y = warp_sum(w_y); w_xy = warp_sum(w_xy); }
+    if (lane == 0) {   // inclusion-exclusion per window bin (index = bx + 2 by); the histogram is private to this warp
+      const unsigned fc[4] = {n_t - n_x - n_y + n_xy, n_x - n_xy, n_y - n_xy, n_xy};
+      const double fs[4] = {(s_t - s_x) - (s_y - s_xy), s_x - s_xy, s_y - s_xy, s_xy};
+      const double fw[4] = {(w_t - w_x) - (w_y - w_xy), w_x - w_xy, w_y - w_xy, w_xy};
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        if (fc[b]) {
+          const int o = (wy0 + (b >> 1)) * nbins + wx0 + (b & 1);
+          my_c[o] += fc[b];
+          my_s[o] += fs[b];
+          if constexpr (WEIGHTED) my_w[o] += fw[b];
+        }
+      }
+    }
+    __syncwarp();
+  }
+  flush_hist(cur_cat);
+  const unsigned long long LEAF = (unsigned long long)PB_CHUNK * PB_CHUNK;
+  if (st_closed) atomicAdd(&g_pb_stats[0], LEAF * st_closed);   // per classifying lane
+  if (lane == 0) {
+    if (st_1d) atomicAdd(&g_pb_stats[1], LEAF * st_1d);
+    if (st_pw) atomicAdd(&g_pb_stats[2], LEAF * st_pw);
+    if (st_sorted) atomicAdd(&g_pb_stats[3], LEAF * st_sorted);
+    if (st_quad) atomicAdd(&g_pb_stats[4], LEAF * st_quad);
+    if (st_pairs) atomicAdd(&g_pb_super_leaves, (unsigned long long)st_pairs);
+  }
+}
+
 extern "C" int tgp_pairbin_tile(void) { return PB_CHUNK; }
 
 // Records of one round of the two-pass TwoD count (16 bytes each): 2^26 = 1 GiB, about 8 rounds at N = 1e6.
@@ -1946,21 +2318,33 @@ static int64_t pb_rec_slots(int64_t max_len, int32_t ncat) {
   if (need >= (double)PB_REC_CAP) return PB_REC_CAP;
   return ((int64_t)need + 255) / 256 * 256;
 }
-// Work buffer of the two-pass count: {3 work counters, 1 spare word} {record counts of a round: slots / 32 ints}
-// {records: 2 doubles each} {pre-pass chunk records} {super-chunk records}.  The other paths keep the chunk records
-// at the start.
-static int64_t pb_rec_region_doubles(int64_t slots) { return 4 + slots / 64 + 2 * slots; }
+// Work buffer of the two-pass count: {work counters of pass A, pass B, the super kernel; length of the TWO_AXIS list,
+// work counter of the leaf kernel; 3 spare words} {record counts of a round: slots / 32 ints} {records: 2 doubles each}
+// {pre-pass chunk records} {super-chunk records} {TWO_AXIS list: 2 doubles per super pair}.  The other paths keep the
+// chunk records at the start.
+static int64_t pb_rec_region_doubles(int64_t slots) { return 8 + slots / 64 + 2 * slots; }
 
 extern "C" int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat) {
+  const int64_t nsup = total_points / PB_SUPER_PTS;   // every catalogue's full super-chunks together
   return pb_rec_region_doubles(pb_rec_slots(total_points, ncat)) +
          (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2) +
-         (int64_t)PB_SUPER_STRIDE * (total_points / PB_SUPER_PTS + (int64_t)ncat + 2);
+         (int64_t)PB_SUPER_STRIDE * (nsup + (int64_t)ncat + 2) + nsup * (nsup > 0 ? nsup - 1 : 0);
 }
 
 static int g_pb_fast_paths = 7;   // tgp_set_option("pairbin_fast_paths", bits): see PBParams::fast_paths
 extern "C" int tgp_pairbin_set_fast_paths(int bits) { g_pb_fast_paths = bits; return TGP_OK; }
 static int g_pb_block_sums = 1;   // tgp_set_option("pairbin_block_sums", 0): every pair evaluated individually
 extern "C" int tgp_pairbin_set_block_sums(int on) { g_pb_block_sums = on ? 1 : 0; return TGP_OK; }
+
+extern "C" int tgp_pairbin_super_leaves(unsigned long long* host1, int reset) {
+  TGP_CHECK_ARG(host1 != nullptr, "host1");
+  TGP_CUDA(cudaMemcpyFromSymbol(host1, g_pb_super_leaves, sizeof(unsigned long long)));
+  if (reset) {
+    const unsigned long long z = 0;
+    TGP_CUDA(cudaMemcpyToSymbol(g_pb_super_leaves, &z, sizeof(z)));
+  }
+  return TGP_OK;
+}
 
 extern "C" int tgp_pairbin_stats(unsigned long long* host8, int reset) {
   TGP_CHECK_ARG(host8 != nullptr, "host8");
@@ -2059,6 +2443,7 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
   P.recs = nullptr;
   P.rec_cnt = nullptr;
   P.counter_next = nullptr;
+  P.slist_len = nullptr;
   if (work) {
     TGP_CHECK_ARG(((uintptr_t)work % 32) == 0, "work must be 32-byte aligned");
     double* bx = work + (split ? pb_rec_region_doubles(rec_slots) : 0);
@@ -2071,12 +2456,13 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
   }
 
   if (split) {
-    // [0] pass A's work counter, [1] pass B's, [2] the super kernel's
+    // [0] pass A's work counter, [1] pass B's, [2] the super kernel's, [3] the TWO_AXIS list length, [4] the leaf
+    // kernel's work counter
     unsigned long long* ctr = reinterpret_cast<unsigned long long*>(work);
-    P.rec_cnt = reinterpret_cast<int*>(work + 4);
-    P.recs = reinterpret_cast<int4*>(work + 4 + rec_slots / 64);
+    P.rec_cnt = reinterpret_cast<int*>(work + 8);
+    P.recs = reinterpret_cast<int4*>(work + 8 + rec_slots / 64);
     const int64_t per_round = (rec_slots < g_pb_rec_cap ? rec_slots : g_pb_rec_cap) / run;   // items
-    TGP_CUDA(cudaMemsetAsync(ctr, 0, 3 * sizeof(unsigned long long), st));
+    TGP_CUDA(cudaMemsetAsync(ctr, 0, 5 * sizeof(unsigned long long), st));
     // super-chunk records (they follow the chunk records; the kernels find them from cat_off[ncat]) and the super
     // kernel, which books the super pairs that the classification pass of every round skips
     // kernel, which books the super pairs that the classification pass of every round skips.  Off when the staging
@@ -2091,6 +2477,7 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
     PS.items_per_cat = nsf_max;   // the super kernel's items of a catalogue: nsf_max rows x runs of 32 columns
     PS.my_items = (super_items - tile_rank + tile_nranks - 1) / tile_nranks;
     PS.counter = ctr + 2;
+    PS.slist_len = ctr + 3;
     PS.warps = warps_s;
     const size_t smem_s = fixed + (size_t)warps_s * per_warp_s + 64;
     if (supers) {
@@ -2111,6 +2498,28 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
       if (grid_s > (int64_t)sms * ctas_s) grid_s = (int64_t)sms * ctas_s;
       if (weighted) pairbin_super_kernel<true><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
       else pairbin_super_kernel<false><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
+      TGP_LAUNCH_CHECK();
+      // the leaf kernel takes the TWO_AXIS super pairs the super kernel listed (the length stays on the device):
+      // warp histograms + one staged column chunk per warp; per_warp_l < per_warp_s, so warps_l >= 1
+      PBParams PL = P;
+      const size_t per_warp_l = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0)) + PB_CHUNK * (16 + 8 + 8);
+      int warps_l = (int)((budget - fixed - 64) / per_warp_l);
+      if (warps_l > PB_MAX_WARPS) warps_l = PB_MAX_WARPS;
+      PL.warps = warps_l;
+      PL.counter = ctr + 4;
+      PL.slist_len = ctr + 3;
+      const size_t smem_l = fixed + (size_t)warps_l * per_warp_l + 64;
+      int ctas_l = (int)((220 * 1024) / smem_l);
+      if (ctas_l > PB_LEAVES_MIN_CTAS) ctas_l = PB_LEAVES_MIN_CTAS;
+      if (ctas_l < 1) ctas_l = 1;
+      static TgpPerDeviceOnce once_l[2];
+      const void* kern_l = weighted ? (const void*)pairbin_super_leaves_kernel<true>
+                                    : (const void*)pairbin_super_leaves_kernel<false>;
+      if (tgp_first_use_on_device(once_l[weighted ? 1 : 0]))
+        TGP_CUDA(cudaFuncSetAttribute(kern_l, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
+      const unsigned grid_l = (unsigned)((int64_t)sms * ctas_l);
+      if (weighted) pairbin_super_leaves_kernel<true><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
+      else pairbin_super_leaves_kernel<false><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
       TGP_LAUNCH_CHECK();
     }
     PBParams PA = P;
