@@ -1982,7 +1982,7 @@ __device__ __forceinline__ bool pb_rank_query_d(const double* __restrict__ xs, d
 }
 
 // Leaf classes inside a TWO_AXIS super pair (pairbin_super_leaves_kernel)
-enum { PB_L_OUT = 0, PB_L_CLOSED = 1, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD = 4, PB_L_PAIRS = 5, PB_L_EDGE = 6 };
+enum { PB_L_OUT = 0, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD = 4, PB_L_PAIRS = 5 };
 
 // The leaf kernel: the TWO_AXIS super pairs of the list, one per warp step (persistent CTAs, device-side counter; the
 // length is read on the device).  A super pair's window [x0, x0 + 1] x [y0, y0 + 1] holds every in-range pair and its
@@ -1994,7 +1994,11 @@ enum { PB_L_OUT = 0, PB_L_CLOSED = 1, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD 
 //   one axis  one rank query per row point on the chunk's copy sorted along the varying axis;
 //   2 x 2     (both windows clean) the column-bit and row-bit sums from two rank queries, the "both bits" quadrant
 //             pair by pair;
-//   otherwise pair by pair over the staged chunk, with the range test where the range edge runs through the block.
+//   otherwise pair by pair over the staged chunk (an unclean mirrored window), with the range test where the range
+//             edge runs through the block.
+// Each axis has one bit per pair, fixed per super pair: the bin edge of the window, or the range edge when the
+// out-of-range region is one of the axis' two slots.  A block the range edge runs through therefore takes the one-axis
+// or 2 x 2 form like any other block whose bit varies; the out-of-range slots are dropped at booking.
 // A failed mirrored-bit check at the split hands the block to the pair-by-pair loop, which counts the pairs whose
 // exact mirrored bin is not the mirror image and moves them in global memory afterwards (as pass B's fix_mirror).
 // The bit predicates compare the displacement fl(c_j - c_i) with the bin thresholds directly (no per-lane coordinate
@@ -2054,6 +2058,7 @@ pairbin_super_leaves_kernel(PBParams P) {
 
   const double M = P.hi, lo2 = P.lo2;
   const int4* slist = pb_super_list(P);
+  const double* sup0 = pb_super_records(P);
   const unsigned long long nlist = *P.slist_len;
   unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0;   // leaf blocks, super pairs
   int cur_cat = -1, since_flush = 0;
@@ -2075,8 +2080,24 @@ pairbin_super_leaves_kernel(PBParams P) {
     const int64_t off = P.cat_off[cat];
     const int64_t r0 = (int64_t)e.y * PB_SUPER, c0 = (int64_t)e.z * PB_SUPER;   // first row / column chunk
     const double* rec0 = P.boxes + (size_t)PB_STRIDE * (size_t)(off / PB_CHUNK + cat);
-    // bits of the window: forward upper bin dx >= tx; the mirrored entry's upper bin -dx >= ed[nbins-1-x0] <=> dx <= mx
-    const double tx = ed[wx0 + 1], ty = ed[wy0 + 1], mx = -ed[nbins - 1 - wx0], my = -ed[nbins - 1 - wy0];
+    // The bit of each axis, fixed per super pair from the super-chunk boxes {xmin, xmax, ymin, ymax} (as
+    // pb_super_status decides): bin edge t = ed[x0 + 1] (bit 0 -> bin x0, bit 1 -> bin x0 + 1); upper range edge
+    // t = max_sep (bit 0 -> bin nbins - 1, bit 1 -> out of range); lower range edge t = the smallest double above
+    // -max_sep (bit 0 -> out, bit 1 -> bin 0).  The mirrored entry's upper bit is d <= m: m = -ed[nbins-1-x0] for a
+    // bin edge; for a range edge m = the double below t, so the mirror check passes by construction (the range test
+    // is the same for both entries, fl(x_i - x_j) = -fl(x_j - x_i), and the in-range mirrored window is the mirror
+    // image).
+    const double4 rsb = *reinterpret_cast<const double4*>(sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat + e.y));
+    const double4 csb = *reinterpret_cast<const double4*>(sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat + e.z));
+    const bool upx = csb.y - rsb.x >= M, lox = csb.x - rsb.y <= -M;
+    const bool upy = csb.w - rsb.z >= M, loy = csb.z - rsb.w <= -M;
+    const double tx = upx ? M : (lox ? nextafter(-M, 0.0) : ed[wx0 + 1]);
+    const double ty = upy ? M : (loy ? nextafter(-M, 0.0) : ed[wy0 + 1]);
+    const double mx = upx ? nextafter(M, 0.0) : (lox ? -M : -ed[nbins - 1 - wx0]);
+    const double my = upy ? nextafter(M, 0.0) : (loy ? -M : -ed[nbins - 1 - wy0]);
+    // forward bin of each bit value, -1 = out of range (dropped at booking)
+    const int bx0 = upx ? nbins - 1 : (lox ? -1 : wx0), bx1 = upx ? -1 : (lox ? 0 : wx0 + 1);
+    const int by0 = upy ? nbins - 1 : (loy ? -1 : wy0), by1 = upy ? -1 : (loy ? 0 : wy0 + 1);
     // the four forward bins of the super pair, per lane: all pairs, x-bit, y-bit, both bits
     unsigned n_t = 0u, n_x = 0u, n_y = 0u, n_xy = 0u;
     double s_t = 0.0, s_x = 0.0, s_y = 0.0, s_xy = 0.0, w_t = 0.0, w_x = 0.0, w_y = 0.0, w_xy = 0.0;
@@ -2092,16 +2113,23 @@ pairbin_super_leaves_kernel(PBParams P) {
       const double4 rb = *reinterpret_cast<const double4*>(rrec);
       int win[4];
       const int cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, cb.x, cb.y, cb.z, cb.w, M, lo2, nbins, ed, win);
-      const int x0 = win[0] & 0xffff, y0 = win[1] & 0xffff, rx0 = win[2] & 0xffff, ry0 = win[3] & 0xffff;
-      const bool one_x = (win[0] >> 16) == 0 && (win[2] >> 16) == 0 && rx0 == nbins - 1 - x0;
-      const bool one_y = (win[1] >> 16) == 0 && (win[3] >> 16) == 0 && ry0 == nbins - 1 - y0;
-      const bool clean_x = (win[0] >> 16) == 1 && (win[2] >> 16) == 1 && rx0 == nbins - 2 - x0;
-      const bool clean_y = (win[1] >> 16) == 1 && (win[3] >> 16) == 1 && ry0 == nbins - 2 - y0;
-      const int bx = x0 - wx0, by = y0 - wy0;   // window bits of an axis in one bin
+      // per axis: 0 / 1 = the bit is constant, 2 = it varies (bin edge with a clean mirrored window, or the range edge
+      // runs through the block), 3 = neither (unclean mirrored window)
+      auto axis = [&](bool up, bool lo, double d0, double d1, int w, int rw, int a) -> int {
+        if (up || lo) return (up ? d1 >= M : d0 <= -M) ? 2 : (up ? 0 : 1);
+        const int x0 = w & 0xffff, rx0 = rw & 0xffff;
+        if ((w >> 16) == 0 && (rw >> 16) == 0 && rx0 == nbins - 1 - x0) return x0 - a;
+        if ((w >> 16) == 1 && (rw >> 16) == 1 && rx0 == nbins - 2 - x0) return 2;
+        return 3;
+      };
+      int bx = 3, by = 3;
+      if (cls == PB_REG_FULL || cls == PB_REG_CHECK) {
+        bx = axis(upx, lox, cb.x - rb.y, cb.y - rb.x, win[0], win[2], wx0);
+        by = axis(upy, loy, cb.z - rb.w, cb.w - rb.z, win[1], win[3], wy0);
+      }
       int c = PB_L_OUT;
-      if (cls == PB_REG_CHECK) c = PB_L_EDGE;
-      else if (cls == PB_REG_FULL) {
-        if (one_x && one_y) {
+      if (cls != PB_OUT) {
+        if (bx < 2 && by < 2) {   // every pair in range, in one slot
           const double2 rs = *reinterpret_cast<const double2*>(rrec + 4);
           const double s = rs.x * cs.x, w = WEIGHTED ? rs.y * cs.y : 0.0;
           const unsigned n = (unsigned)(PB_CHUNK * PB_CHUNK);
@@ -2110,9 +2138,10 @@ pairbin_super_leaves_kernel(PBParams P) {
           if (by) { n_y += n; s_y += s; w_y += w; }
           if (bx && by) { n_xy += n; s_xy += s; w_xy += w; }
           ++st_closed;
-        } else if (one_y) c = PB_L_ONE_X | (by << 3);      // x varies, the y bit is constant
-        else if (one_x) c = PB_L_ONE_Y | (bx << 3);
-        else c = (clean_x && clean_y && (P.fast_paths & 2)) ? PB_L_QUAD : PB_L_PAIRS;
+        } else if (bx == 2 && by < 2) c = PB_L_ONE_X | (by << 3);   // x varies, the y bit is constant
+        else if (by == 2 && bx < 2) c = PB_L_ONE_Y | (bx << 3);
+        else c = (bx == 2 && by == 2 && (P.fast_paths & 2)) ? PB_L_QUAD : PB_L_PAIRS;
+        if (cls != PB_REG_FULL && c != PB_L_OUT) c |= 16;   // the range edge runs through the block
       }
       code[h] = c;
     }
@@ -2155,12 +2184,13 @@ pairbin_super_leaves_kernel(PBParams P) {
         const int c = __ffs(m) - 1;
         m &= m - 1;
         const int lc = __shfl_sync(0xffffffffu, codes, (rk & 3) * 8 + c);
-        const int cls = lc & 7, cbit = lc >> 3;
+        const int cls = lc & 7, cbit = (lc >> 3) & 1;
+        const bool check = (lc >> 4) & 1;
         const double csk = __shfl_sync(0xffffffffu, cs.x, c);
         double csw = 0.0;
         if constexpr (WEIGHTED) csw = __shfl_sync(0xffffffffu, cs.y, c);
         const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + c) + PB_SLOT;   // sorted copies of the chunk
-        bool per_pair = cls >= PB_L_PAIRS;
+        bool per_pair = cls == PB_L_PAIRS;
         if (cls == PB_L_ONE_X || cls == PB_L_ONE_Y) {
           const bool vx = cls == PB_L_ONE_X;
           const double* xs = vx ? srt : srt + 3 * PB_CHUNK;
@@ -2218,11 +2248,10 @@ pairbin_super_leaves_kernel(PBParams P) {
           per_pair = true;
         }
         if (!per_pair) continue;
-        // pair by pair over the raw points of the chunk: every in-range pair sits in the window; EDGE blocks test the
-        // range per pair (r2 >= lo2 holds for every pair of a TWO_AXIS super pair)
+        // pair by pair over the raw points of the chunk: every in-range pair sits in the window; blocks the range edge
+        // runs through test the range per pair (r2 >= lo2 holds for every pair of a TWO_AXIS super pair)
         if (cls != PB_L_ONE_X && cls != PB_L_ONE_Y) ++st_pw;
         stage(c);
-        const bool check = cls == PB_L_EDGE;
         unsigned mmc = 0u;
         double a_t = 0.0, a_x = 0.0, a_y = 0.0, a_xy = 0.0, b_t = 0.0, b_x = 0.0, b_y = 0.0, b_xy = 0.0;
 #pragma unroll 2
@@ -2251,8 +2280,11 @@ pairbin_super_leaves_kernel(PBParams P) {
             if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
             const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
             if ((px != qx) && (py != qy)) continue;
-            const int assumed = (nbins - 1 - (wy0 + (py ? 1 : 0))) * nbins + (nbins - 1 - (wx0 + (px ? 1 : 0)));
-            const int exact = (nbins - 2 - wy0 + (qy ? 1 : 0)) * nbins + (nbins - 2 - wx0 + (qx ? 1 : 0));
+            // only bin-edge bits can disagree; a range bit's mirrored bin is the mirror image
+            const int fx = px ? bx1 : bx0, fy = py ? by1 : by0;
+            const int ex = px != qx ? nbins - 1 - fx : nbins - 2 - wx0 + (qx ? 1 : 0);
+            const int ey = py != qy ? nbins - 1 - fy : nbins - 2 - wy0 + (qy ? 1 : 0);
+            const int assumed = (nbins - 1 - fy) * nbins + (nbins - 1 - fx), exact = ey * nbins + ex;
             const double kk = ki * ck[jj];
             double ww = 1.0;
             if constexpr (WEIGHTED) ww = wi * cw[jj];
@@ -2271,14 +2303,15 @@ pairbin_super_leaves_kernel(PBParams P) {
     n_t = warp_sum_u(n_t); n_x = warp_sum_u(n_x); n_y = warp_sum_u(n_y); n_xy = warp_sum_u(n_xy);
     s_t = warp_sum(s_t); s_x = warp_sum(s_x); s_y = warp_sum(s_y); s_xy = warp_sum(s_xy);
     if constexpr (WEIGHTED) { w_t = warp_sum(w_t); w_x = warp_sum(w_x); w_y = warp_sum(w_y); w_xy = warp_sum(w_xy); }
-    if (lane == 0) {   // inclusion-exclusion per window bin (index = bx + 2 by); the histogram is private to this warp
+    if (lane == 0) {   // inclusion-exclusion per slot (index = bx + 2 by), out-of-range slots dropped; private histogram
       const unsigned fc[4] = {n_t - n_x - n_y + n_xy, n_x - n_xy, n_y - n_xy, n_xy};
       const double fs[4] = {(s_t - s_x) - (s_y - s_xy), s_x - s_xy, s_y - s_xy, s_xy};
       const double fw[4] = {(w_t - w_x) - (w_y - w_xy), w_x - w_xy, w_y - w_xy, w_xy};
 #pragma unroll
       for (int b = 0; b < 4; ++b) {
-        if (fc[b]) {
-          const int o = (wy0 + (b >> 1)) * nbins + wx0 + (b & 1);
+        const int fx = (b & 1) ? bx1 : bx0, fy = (b >> 1) ? by1 : by0;
+        if (fc[b] && fx >= 0 && fy >= 0) {
+          const int o = fy * nbins + fx;
           my_c[o] += fc[b];
           my_s[o] += fs[b];
           if constexpr (WEIGHTED) my_w[o] += fw[b];
