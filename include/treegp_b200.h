@@ -481,6 +481,10 @@ int tgp_pairbin_stats(unsigned long long* host8 /*host*/, int reset);
  * bins per axis (the range edge counting as one) and had their 32-point blocks decided by the leaf kernel without
  * block records.  Their blocks are tallied in the slots of tgp_pairbin_stats as usual.  Synchronous. */
 int tgp_pairbin_super_leaves(unsigned long long* host1 /*host*/, int reset);
+/* Diagnostics: how many of those super-chunk pairs were decided per row point against the column super-chunk staged
+ * in shared memory (the others went block by block, after a failed mirrored-bit check or when the staged tables do not
+ * fit).  Synchronous. */
+int tgp_pairbin_super_rows(unsigned long long* host1 /*host*/, int reset);
 
 /* Test and measurement switches of the pair counts (tgp_pairbin_*, tgp_bootbin_twod), not needed for normal use.
  * Any other name is rejected with TGP_ERR_INVALID ("unknown option").

@@ -712,9 +712,9 @@ _PB_SCRATCH = {}
 
 
 def _pairbin_scratch(dev, doubles):
-    """The workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6, the super-chunk records and
-    the list of super pairs for the leaf kernel, ~170 MB, plus the block records of one round of the two-pass TwoD
-    count, at most 1 GiB), kept per
+    """The workspace of tgp_pairbin (chunk boxes + sorted chunk copies, ~50 MB at N = 1e6, the super-chunk records, the
+    list of super pairs for the leaf kernel and the same list grouped by column super-chunk, ~300 MB, plus the block
+    records of one round of the two-pass TwoD count, at most 1 GiB), kept per
     (device, stream) and grown on demand: launches on one stream are ordered, so they can share it; launches on
     different streams get different buffers."""
     key = (dev.index, torch.cuda.current_stream(dev).cuda_stream)
@@ -877,6 +877,14 @@ def pairbin_super_leaves(reset=True):
     apart from pairbin_stats, whose values are pair counts that add up to the total."""
     v = ctypes.c_ulonglong(0)
     check(_cabi.load().tgp_pairbin_super_leaves(ctypes.byref(v), int(bool(reset))), "tgp_pairbin_super_leaves")
+    return int(v.value)
+
+
+def pairbin_super_rows(reset=True):
+    """Of the super-chunk pairs of pairbin_super_leaves, those decided per row point against the staged column
+    super-chunk (see tgp_pairbin_super_rows)."""
+    v = ctypes.c_ulonglong(0)
+    check(_cabi.load().tgp_pairbin_super_rows(ctypes.byref(v), int(bool(reset))), "tgp_pairbin_super_rows")
     return int(v.value)
 
 

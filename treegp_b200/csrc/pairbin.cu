@@ -28,9 +28,10 @@
 // of the residual paths, so it runs at more warps per SM and the residual kernel's warm code no longer contains it.
 // Before the rounds, pairbin_super_kernel books the pairs of super-chunks (PB_SUPER chunks) that are out of range, sit
 // in one bin, or vary along one axis only (one rank query per row point on the super-chunk's sorted copy), and lists
-// those that span at most 2 x 2 bins; pairbin_super_leaves_kernel decides the 32-point blocks of the listed pairs in
-// one launch, without records.  The classification pass skips the blocks of all of them and descends to the 32-point
-// blocks only for the other super pairs.
+// those that span at most 2 x 2 bins; pairbin_super_leaves_kernel decides the listed pairs in one launch, without
+// records: per row point against the column super-chunk staged in shared memory (the list grouped by column
+// super-chunk), or block by block.  The classification pass skips the blocks of all of them and descends to the
+// 32-point blocks only for the other super pairs.
 //
 // Two instantiations per bin type (template parameter BS):
 //   BS = false  the pair-by-pair kernel: every pair of every in-range block is evaluated individually
@@ -1475,6 +1476,42 @@ __device__ __forceinline__ int4* pb_super_list(const PBParams& P) {
   return reinterpret_cast<int4*>(const_cast<double*>(pb_super_records(P)) +
                                  (size_t)PB_SUPER_STRIDE * (size_t)(P.cat_off[P.ncat] / PB_SUPER_PTS + P.ncat + 2));
 }
+
+// Super pairs per work item of the staged leaf kernel: a slice of the TWO_AXIS pairs that share a column super-chunk.
+// 128 measured best overall on a B200 (DESIGN section 5, v13): 256 builds fewer tables but balances worse at N = 2e5.
+constexpr int PB_LEAF_SLICE = 128;
+// Entries of the TWO_AXIS list (every super pair of every catalogue), super-chunk slots, and work items of the grouped
+// list (at most one partial slice per slot), from the total point count.
+__host__ __device__ __forceinline__ int64_t pb_super_list_cap(int64_t total) {
+  const int64_t nsup = total / PB_SUPER_PTS;
+  return nsup * (nsup > 0 ? nsup - 1 : 0) / 2;
+}
+__host__ __device__ __forceinline__ int64_t pb_super_slots(int64_t total, int32_t ncat) {
+  return total / PB_SUPER_PTS + ncat + 2;
+}
+__host__ __device__ __forceinline__ int64_t pb_super_items_cap(int64_t total, int32_t ncat) {
+  return (pb_super_list_cap(total) / PB_LEAF_SLICE + pb_super_slots(total, ncat) + 1) & ~(int64_t)1;
+}
+// Behind the TWO_AXIS list: the links of the super-chunk records (PB_SUPER_PTS halfwords per slot: for every x-sorted
+// position, the point's index in the super-chunk | its position in the stored y-sorted copy << 8), one word per slot
+// (TWO_AXIS pairs with that column super-chunk, then their offset in the grouped list), the work items {first entry
+// << 16 | entries} and the list grouped by column super-chunk.  `boxes` = the chunk records.
+struct PBSuperGroups {
+  unsigned short* links;
+  unsigned long long *goff, *items;
+  int4* glist;
+};
+__device__ __forceinline__ PBSuperGroups pb_super_groups(const double* boxes, const int64_t* cat_off, int32_t ncat) {
+  const int64_t total = cat_off[ncat], nslot = pb_super_slots(total, ncat);
+  const double* rec = boxes + (size_t)PB_STRIDE * (size_t)(total / PB_CHUNK + ncat + 2);
+  PBSuperGroups g;
+  g.links = reinterpret_cast<unsigned short*>(const_cast<int4*>(
+      reinterpret_cast<const int4*>(rec + (size_t)PB_SUPER_STRIDE * (size_t)nslot) + pb_super_list_cap(total)));
+  g.goff = reinterpret_cast<unsigned long long*>(g.links + (size_t)PB_SUPER_PTS * nslot);
+  g.items = g.goff + ((nslot + 1) & ~(int64_t)1);
+  g.glist = reinterpret_cast<int4*>(g.items + pb_super_items_cap(total, ncat));
+  return g;
+}
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_CLASSIFY_MIN_CTAS)
 pairbin_classify_kernel(PBParams P) {
@@ -1708,13 +1745,23 @@ pairbin_boxes_kernel(const double* __restrict__ px, const double* __restrict__ p
 // (bitonic network in shared memory) and stores them with the suffix sums of k w and w, the box (the sorted ends) and
 // the sums (the first suffix sums of the x order).  Record of super-chunk s of catalogue `cat`:
 // PB_SUPER_STRIDE x (cat_off[cat] / PB_SUPER_PTS + s + cat) doubles from the start of the super records, which
-// follow the chunk records (`boxes`).
+// follow the chunk records (`boxes`).  The point index is carried through both sorts, so the links (pb_super_groups)
+// name, for every x-sorted position, the point and its position in the y-sorted copy as stored.  The CTAs also zero
+// the group counts of every slot.
 __global__ void __launch_bounds__(PB_SUPER_PTS)
 pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restrict__ py, const double* __restrict__ pk,
                            const double* __restrict__ pw, const int64_t* __restrict__ cat_off, int32_t ncat,
                            int64_t supers_per_cat, double* __restrict__ boxes) {
   __shared__ double s_key[PB_SUPER_PTS], s_k[PB_SUPER_PTS], s_w[PB_SUPER_PTS], s_part[2][PB_SUPER_PTS / 32];
+  __shared__ int s_idx[PB_SUPER_PTS];
+  __shared__ unsigned char s_xi[PB_SUPER_PTS], s_yr[PB_SUPER_PTS];
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  {
+    unsigned long long* goff = pb_super_groups(boxes, cat_off, ncat).goff;
+    const int64_t nslot = pb_super_slots(cat_off[ncat], ncat);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + t; i < nslot; i += (int64_t)gridDim.x * blockDim.x)
+      goff[i] = 0ull;
+  }
   const int64_t cat = blockIdx.x / supers_per_cat, s = blockIdx.x % supers_per_cat;
   if (cat >= ncat) return;
   const int64_t off = cat_off[cat], n = cat_off[cat + 1] - off;
@@ -1727,6 +1774,7 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
     s_key[t] = axis == 0 ? px[j] : py[j];
     s_k[t] = kj;
     s_w[t] = wj;
+    s_idx[t] = t;
     __syncthreads();
     for (int k2 = 2; k2 <= PB_SUPER_PTS; k2 <<= 1) {
       for (int j2 = k2 >> 1; j2 > 0; j2 >>= 1) {
@@ -1737,6 +1785,7 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
             double v = s_key[t]; s_key[t] = s_key[u]; s_key[u] = v;
             v = s_k[t]; s_k[t] = s_k[u]; s_k[u] = v;
             v = s_w[t]; s_w[t] = s_w[u]; s_w[u] = v;
+            const int iv = s_idx[t]; s_idx[t] = s_idx[u]; s_idx[u] = iv;
           }
         }
         __syncthreads();
@@ -1761,6 +1810,14 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
       o[2 * axis + 1] = s_key[PB_SUPER_PTS - 1];
       if (axis == 0) { o[4] = vk; o[5] = vw; o[6] = 0.0; o[7] = 0.0; }
     }
+    if (axis == 0) {
+      s_xi[t] = (unsigned char)s_idx[t];   // x position t holds point s_idx[t]
+    } else {
+      s_yr[s_idx[t]] = (unsigned char)t;   // point s_idx[t] sits at y position t
+      __syncthreads();
+      pb_super_groups(boxes, cat_off, ncat).links[(size_t)PB_SUPER_PTS * (size_t)(off / PB_SUPER_PTS + s + cat) + t] =
+          (unsigned short)(s_xi[t] | (s_yr[s_xi[t]] << 8));
+    }
     __syncthreads();   // the buffers are refilled for the y order
   }
 }
@@ -1774,7 +1831,7 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
 //             predicate (monotone in c_j).  The upper bin gets n_C - pos pairs and k_i w_i x suffix(pos), the lower bin
 //             the rest.  The exact mirrored bits differ from the mirror image only for the columns between pos and
 //             pos_m = #{j : fl(c_j - c_i) <= -t_m}, nearly always none; those pairs are moved in global memory.
-//   TWO_AXIS  appended to the list of the leaf kernel (pairbin_super_leaves_kernel).
+//   TWO_AXIS  appended to the list of the leaf kernel (pairbin_super_leaves_kernel) and counted per column super-chunk.
 // The warp histograms hold forward entries; the mirror image is added when they are written out.
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, 2)
@@ -1827,6 +1884,7 @@ pairbin_super_kernel(PBParams P) {
   const double M = P.hi, lo2 = P.lo2;
   const double* sup0 = pb_super_records(P);
   int4* slist = pb_super_list(P);
+  unsigned long long* goff = pb_super_groups(P.boxes, P.cat_off, P.ncat).goff;
   const int64_t nruns = (P.items_per_cat + 31) / 32;   // items_per_cat: super-chunks of the longest catalogue
   unsigned st_closed = 0, st_one = 0;   // super pairs
   int cur_cat = -1, since_flush = 0;
@@ -1860,8 +1918,10 @@ pairbin_super_kernel(PBParams P) {
       unsigned long long base = 0;
       if (lane == 0) base = atomicAdd(P.slist_len, (unsigned long long)__popc(two));
       base = __shfl_sync(0xffffffffu, base, 0);
-      if (st == PB_S_TWO_AXIS)
+      if (st == PB_S_TWO_AXIS) {
         slist[base + __popc(two & ((1u << lane) - 1u))] = make_int4(cat, (int)R, (int)C, x0 | (y0 << 16));
+        atomicAdd(goff + off / PB_SUPER_PTS + cat + C, 1ull);   // group size of column super-chunk C
+      }
     }
     if (st == PB_S_CLOSED) {
       const double2 csum = *reinterpret_cast<const double2*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)C + 4);
@@ -1966,8 +2026,58 @@ pairbin_super_kernel(PBParams P) {
   if (st_one) atomicAdd(&g_pb_stats[6], (unsigned long long)PB_SUPER_PTS * PB_SUPER_PTS * st_one);
 }
 
-// Super pairs taken by the leaf kernel since the last reset (tgp_pairbin_super_leaves).  Diagnostics.
+// Super pairs taken by the leaf kernel since the last reset (tgp_pairbin_super_leaves), and those of them decided per row
+// point against the staged column super-chunk (tgp_pairbin_super_rows).  Diagnostics.
 __device__ unsigned long long g_pb_super_leaves;
+__device__ unsigned long long g_pb_super_rows;
+
+// Grouping of the TWO_AXIS list by column super-chunk, for the staged leaf kernel (one CTA): the group sizes counted by
+// the super kernel become offsets (exclusive scan over the slots), and every group is cut into work items of at most
+// PB_LEAF_SLICE entries.  The number of items goes to work word 5 (P.slist_len[2]); the host never reads it.
+__global__ void __launch_bounds__(1024) pairbin_super_group_kernel(PBParams P) {
+  __shared__ unsigned long long s_part[2][32];
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
+  const int64_t nslot = pb_super_slots(P.cat_off[P.ncat], P.ncat);
+  const int64_t per = (nslot + blockDim.x - 1) / blockDim.x;
+  const int64_t s0 = min((int64_t)t * per, nslot), s1 = min(s0 + per, nslot);
+  unsigned long long c = 0, m = 0;
+  for (int64_t s = s0; s < s1; ++s) {
+    const unsigned long long v = grp.goff[s];
+    c += v;
+    m += (v + PB_LEAF_SLICE - 1) / PB_LEAF_SLICE;
+  }
+  unsigned long long ic = c, im = m;   // inclusive scans over the warp, then over the warps
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned long long tc = __shfl_up_sync(0xffffffffu, ic, o), tm = __shfl_up_sync(0xffffffffu, im, o);
+    if (lane >= o) { ic += tc; im += tm; }
+  }
+  if (lane == 31) { s_part[0][warp] = ic; s_part[1][warp] = im; }
+  __syncthreads();
+  for (int u = 0; u < warp; ++u) { ic += s_part[0][u]; im += s_part[1][u]; }
+  unsigned long long o = ic - c, io = im - m;
+  for (int64_t s = s0; s < s1; ++s) {
+    const unsigned long long v = grp.goff[s];
+    grp.goff[s] = o;
+    for (unsigned long long k = 0; k < v; k += PB_LEAF_SLICE)
+      grp.items[io++] = ((o + k) << 16) | (v - k < PB_LEAF_SLICE ? v - k : (unsigned long long)PB_LEAF_SLICE);
+    o += v;
+  }
+  if (t == (int)blockDim.x - 1) P.slist_len[2] = io;
+}
+
+// Scatter of the TWO_AXIS list into its groups (the order inside a group is immaterial).
+__global__ void __launch_bounds__(256) pairbin_super_scatter_kernel(PBParams P) {
+  const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
+  const int4* slist = pb_super_list(P);
+  const unsigned long long n = *P.slist_len;
+  for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+       i += (unsigned long long)gridDim.x * blockDim.x) {
+    const int4 e = slist[i];
+    grp.glist[atomicAdd(grp.goff + P.cat_off[e.x] / PB_SUPER_PTS + e.x + e.z, 1ull)] = e;
+  }
+}
 
 // Rank query with the bin predicate on the displacement itself: pos = #{j : fl(c_j - ci) < t} in a chunk's ascending
 // copy xs (4-ary search as pb_rank_query_g: 3 + 3 + 2 probes in three dependent steps).  fl(c_j - ci) is monotone in
@@ -1984,11 +2094,104 @@ __device__ __forceinline__ bool pb_rank_query_d(const double* __restrict__ xs, d
 // Leaf classes inside a TWO_AXIS super pair (pairbin_super_leaves_kernel)
 enum { PB_L_OUT = 0, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD = 4, PB_L_PAIRS = 5 };
 
-// The leaf kernel: the TWO_AXIS super pairs of the list, one per warp step (persistent CTAs, device-side counter; the
-// length is read on the device).  A super pair's window [x0, x0 + 1] x [y0, y0 + 1] holds every in-range pair and its
-// mirrored window is the mirror image, so the lanes keep four forward bins in registers for the whole super pair
-// (sums over all pairs, over the x-bit, the y-bit and both bits; inclusion-exclusion at the end).  Its 64 leaf blocks
-// (32 x 32 points) are decided as pass B decides them, from pb_classify_twod on the chunk boxes of the pre-pass:
+// The bit of each axis of a TWO_AXIS super pair, fixed per super pair from the super-chunk boxes {xmin, xmax, ymin,
+// ymax} of rows (rsb) and columns (csb), as pb_super_status decides: bin edge t = ed[x0 + 1] (bit 0 -> bin x0, bit 1
+// -> bin x0 + 1); upper range edge t = max_sep (bit 0 -> bin nbins - 1, bit 1 -> out of range); lower range edge t =
+// the smallest double above -max_sep (bit 0 -> out, bit 1 -> bin 0).  The mirrored entry's upper bit is d <= m: m =
+// -ed[nbins-1-x0] for a bin edge; for a range edge m = the double below t, so the mirror check passes by construction
+// (the range test is the same for both entries, fl(x_i - x_j) = -fl(x_j - x_i), and the in-range mirrored window is
+// the mirror image).  b*0 / b*1 = forward bin of each bit value, -1 = out of range (dropped at booking).
+struct PBLeafBits {
+  double tx, ty, mx, my;
+  int bx0, bx1, by0, by1;
+  bool upx, lox, upy, loy;
+};
+__device__ __forceinline__ PBLeafBits pb_leaf_bits(const double4& rsb, const double4& csb, double M, int nbins,
+                                                   const double* __restrict__ ed, int wx0, int wy0) {
+  PBLeafBits b;
+  b.upx = csb.y - rsb.x >= M;
+  b.lox = csb.x - rsb.y <= -M;
+  b.upy = csb.w - rsb.z >= M;
+  b.loy = csb.z - rsb.w <= -M;
+  b.tx = b.upx ? M : (b.lox ? nextafter(-M, 0.0) : ed[wx0 + 1]);
+  b.ty = b.upy ? M : (b.loy ? nextafter(-M, 0.0) : ed[wy0 + 1]);
+  b.mx = b.upx ? nextafter(M, 0.0) : (b.lox ? -M : -ed[nbins - 1 - wx0]);
+  b.my = b.upy ? nextafter(M, 0.0) : (b.loy ? -M : -ed[nbins - 1 - wy0]);
+  b.bx0 = b.upx ? nbins - 1 : (b.lox ? -1 : wx0);
+  b.bx1 = b.upx ? -1 : (b.lox ? 0 : wx0 + 1);
+  b.by0 = b.upy ? nbins - 1 : (b.loy ? -1 : wy0);
+  b.by1 = b.upy ? -1 : (b.loy ? 0 : wy0 + 1);
+  return b;
+}
+
+// The staged column super-chunk of the leaf kernel.  With p_x = #{j : x-bit 0} (a split of the x-sorted copy) and p_y
+// the same on the y-sorted copy, the "both bits" quadrant {j : x position >= p_x, y position >= p_y} is read from a
+// two-level dominance table over x-blocks of PB_LT_XB consecutive x positions:
+//   U[b][p_y]      sum k w, sum w (uk, uw) and count (uc) over x-blocks >= b with y position >= p_y (row NB = 0);
+//   Qr[b][p_y]     members of x-block b with y position < p_y;
+//   V[b][xo][q]    sum k w, sum w over members of x-block b with in-block x offset >= xo and in-block y order >= q;
+//   msk[b][q]      the members of x-block b with in-block y order >= q, as a bit mask over the x offsets;
+// quadrant = U[b + 1][p_y] + V[b][p_x % XB][Qr[b][p_y]] with b = p_x / XB (empty for p_x = PB_SUPER_PTS), its count
+// U[b + 1][p_y] + popc(msk[b][Qr[b][p_y]] >> (p_x % XB)).  Suffix sums of the two sorted copies give the x-bit and
+// the y-bit sums; index PB_SUPER_PTS of every suffix array is 0.  kx, wx, yr, xp, yo: k w and w in x order, the y
+// position of every x position and its inverse, the in-block y order (build only).
+constexpr int PB_LT_XB = 16, PB_LT_NB = PB_SUPER_PTS / PB_LT_XB, PB_LT_N = PB_SUPER_PTS + 1;
+constexpr int PB_LT_U = (PB_LT_NB + 1) * PB_LT_N, PB_LT_V = PB_LT_NB * PB_LT_XB * (PB_LT_XB + 1);
+__host__ __device__ constexpr size_t pb_leaf_table_doubles(bool w) {
+  return ((size_t)(w ? 2 : 1) * (2 * PB_LT_N + PB_LT_U + PB_LT_V + PB_SUPER_PTS) + 2 * PB_SUPER_PTS + 1) & ~(size_t)1;
+}
+constexpr size_t PB_LT_TAIL =   // msk, uc, qr, yr, xp, yo (bytes, 16-byte multiple)
+    ((size_t)PB_LT_NB * (PB_LT_XB + 1) * 4 + ((size_t)PB_LT_U * 2 + 3) / 4 * 4 + (size_t)PB_LT_NB * PB_LT_N +
+     3 * PB_SUPER_PTS + 15) / 16 * 16;
+__host__ __device__ constexpr size_t pb_leaf_table_bytes(bool w) { return pb_leaf_table_doubles(w) * 8 + PB_LT_TAIL; }
+struct PBLeafTable {
+  double *xs, *ys, *sxk, *syk, *sxw, *syw, *uk, *uw, *vk, *vw, *kx, *wx;
+  unsigned* msk;
+  unsigned short* uc;
+  unsigned char *qr, *yr, *xp, *yo;
+  __device__ __forceinline__ void carve(double* p, bool w) {
+    double* q = p;
+    xs = q; q += PB_SUPER_PTS;
+    ys = q; q += PB_SUPER_PTS;
+    sxk = q; q += PB_LT_N;
+    syk = q; q += PB_LT_N;
+    uk = q; q += PB_LT_U;
+    vk = q; q += PB_LT_V;
+    kx = q; q += PB_SUPER_PTS;
+    sxw = syw = uw = vw = wx = nullptr;
+    if (w) {
+      sxw = q; q += PB_LT_N;
+      syw = q; q += PB_LT_N;
+      uw = q; q += PB_LT_U;
+      vw = q; q += PB_LT_V;
+      wx = q;
+    }
+    msk = reinterpret_cast<unsigned*>(p + pb_leaf_table_doubles(w));
+    uc = reinterpret_cast<unsigned short*>(msk + PB_LT_NB * (PB_LT_XB + 1));
+    qr = reinterpret_cast<unsigned char*>(uc) + (PB_LT_U * 2 + 3) / 4 * 4;
+    yr = qr + PB_LT_NB * PB_LT_N;
+    xp = yr + PB_SUPER_PTS;
+    yo = xp + PB_SUPER_PTS;
+  }
+};
+
+// The leaf kernel: the TWO_AXIS super pairs of the list.  A super pair's window [x0, x0 + 1] x [y0, y0 + 1] holds every
+// in-range pair and its mirrored window is the mirror image, so the lanes keep four forward bins in registers for the
+// whole super pair (sums over all pairs, over the x-bit, the y-bit and both bits; inclusion-exclusion at the end).
+// Each axis has one bit per pair, fixed per super pair (pb_leaf_bits).
+//
+// STAGED (the default when the tables fit in shared memory): work items are slices of the list grouped by column
+// super-chunk C (pairbin_super_group_kernel).  A CTA claims an item, stages C's sorted copies and the dominance table
+// (PBLeafTable) once, and its warps pull the slice's super pairs from a shared counter.  For each of the 256 row points
+// of a super pair, p_x and p_y come from bisections on the staged copies and the four sums from the suffix sums and the
+// table; the exact mirrored bits need only the neighbours of each split.  If any check fails (a column within rounding
+// of a bin edge), the super pair goes through the per-block body below instead.  One histogram per CTA, booked with
+// shared atomics once per super pair, written out when the catalogue changes and at the end.
+//
+// Otherwise one super pair per warp step from the list itself (device-side counter), warp histograms, per-block body.
+//
+// The per-block body decides the 64 leaf blocks (32 x 32 points) as pass B decides them, from pb_classify_twod on the
+// chunk boxes of the pre-pass:
 //   closed    in ONE bin whose mirrored window is its mirror image: booked by the classifying lane (2 blocks per lane)
 //             from the chunk sums, no point loaded;
 //   one axis  one rank query per row point on the chunk's copy sorted along the varying axis;
@@ -1996,18 +2199,18 @@ enum { PB_L_OUT = 0, PB_L_ONE_X = 2, PB_L_ONE_Y = 3, PB_L_QUAD = 4, PB_L_PAIRS =
 //             pair by pair;
 //   otherwise pair by pair over the staged chunk (an unclean mirrored window), with the range test where the range
 //             edge runs through the block.
-// Each axis has one bit per pair, fixed per super pair: the bin edge of the window, or the range edge when the
-// out-of-range region is one of the axis' two slots.  A block the range edge runs through therefore takes the one-axis
-// or 2 x 2 form like any other block whose bit varies; the out-of-range slots are dropped at booking.
-// A failed mirrored-bit check at the split hands the block to the pair-by-pair loop, which counts the pairs whose
-// exact mirrored bin is not the mirror image and moves them in global memory afterwards (as pass B's fix_mirror).
-// The bit predicates compare the displacement fl(c_j - c_i) with the bin thresholds directly (no per-lane coordinate
-// thresholds).  The warp histograms hold forward entries; the mirror image is added when they are written out.
+// A block the range edge runs through takes the one-axis or 2 x 2 form like any other block whose bit varies; the
+// out-of-range slots are dropped at booking.  A failed mirrored-bit check at the split hands the block to the
+// pair-by-pair loop, which counts the pairs whose exact mirrored bin is not the mirror image and moves them in global
+// memory afterwards (as pass B's fix_mirror).  The blocks of a super pair decided per row point are classified all
+// the same and attributed to the path statistics by their form class.
+// The bit predicates compare the displacement fl(c_j - c_i) with the thresholds directly (no per-lane coordinate
+// thresholds).  The histograms hold forward entries; the mirror image is added when they are written out.
 #ifndef PB_LEAVES_MIN_CTAS
 #define PB_LEAVES_MIN_CTAS 2
 #endif
-template <bool WEIGHTED>
-__global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_LEAVES_MIN_CTAS)
+template <bool WEIGHTED, bool STAGED>
+__global__ void __launch_bounds__(PB_MAX_WARPS * 32 * (STAGED ? 2 : 1), STAGED ? 1 : PB_LEAVES_MIN_CTAS)
 pairbin_super_leaves_kernel(PBParams P) {
   extern __shared__ __align__(16) unsigned char pb_smem[];
   const int nb = P.nb, nbins = P.nbins;
@@ -2016,20 +2219,32 @@ pairbin_super_leaves_kernel(PBParams P) {
   double2* cxy_all = reinterpret_cast<double2*>(ed + ((nbins + 2) & ~1));   // [warps][32]
   double* ck_all = reinterpret_cast<double*>(cxy_all + P.warps * PB_CHUNK);  // [warps][32]
   double* cw_all = ck_all + P.warps * PB_CHUNK;                              // [warps][32]
-  double* hs_all = cw_all + P.warps * PB_CHUNK;                              // [warps][nb]  sum wk wk
-  double* hw_all = hs_all + (size_t)P.warps * nb;                            // [warps][nb]  sum w w     (WEIGHTED)
-  unsigned* hc_all = reinterpret_cast<unsigned*>(hw_all + (WEIGHTED ? (size_t)P.warps * nb : 0));
+  // !STAGED: [warps][nb] sum wk wk, sum w w (WEIGHTED), counts (32 bit); STAGED: [nb] of each, counts 64 bit
+  double* hs_all = cw_all + P.warps * PB_CHUNK;
+  double* hw_all = hs_all + (size_t)(STAGED ? 1 : P.warps) * nb;
+  unsigned* hc_all = reinterpret_cast<unsigned*>(hw_all + (WEIGHTED ? (size_t)(STAGED ? 1 : P.warps) * nb : 0));
+  unsigned long long* hc_cta = reinterpret_cast<unsigned long long*>(hc_all);
   double2* cxy = cxy_all + warp * PB_CHUNK;
   double* ck = ck_all + warp * PB_CHUNK;
   double* cw = cw_all + warp * PB_CHUNK;
-  double* my_s = hs_all + (size_t)warp * nb;
-  double* my_w = hw_all + (size_t)warp * nb;
+  double* my_s = hs_all + (size_t)(STAGED ? 0 : warp) * nb;
+  double* my_w = hw_all + (size_t)(STAGED ? 0 : warp) * nb;
   unsigned* my_c = hc_all + (size_t)warp * nb;
+  PBLeafTable T;
+  if constexpr (STAGED) T.carve(reinterpret_cast<double*>(hc_cta + nb), WEIGHTED);
   for (int i = tid; i <= nbins; i += blockDim.x) ed[i] = P.edges[i];
-  for (int i = lane; i < nb; i += 32) {
-    my_s[i] = 0.0;
-    my_c[i] = 0u;
-    if constexpr (WEIGHTED) my_w[i] = 0.0;
+  if constexpr (STAGED) {
+    for (int i = tid; i < nb; i += blockDim.x) {
+      my_s[i] = 0.0;
+      hc_cta[i] = 0ull;
+      if constexpr (WEIGHTED) my_w[i] = 0.0;
+    }
+  } else {
+    for (int i = lane; i < nb; i += 32) {
+      my_s[i] = 0.0;
+      my_c[i] = 0u;
+      if constexpr (WEIGHTED) my_w[i] = 0.0;
+    }
   }
   __syncthreads();
 
@@ -2055,272 +2270,496 @@ pairbin_super_leaves_kernel(PBParams P) {
     }
     __syncwarp();
   };
+  auto flush_cta = [&](int cat) {   // the same for the CTA histogram (all threads, after a CTA barrier)
+    if (cat < 0) return;
+    for (int b = tid; b < nb; b += blockDim.x) {
+      const int bm = nb - 1 - b;
+      const unsigned long long c = hc_cta[b] + hc_cta[bm];
+      if (c) {
+        const size_t o = (size_t)cat * nb + b;
+        atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + o, c);
+        atomicAdd(P.sumwkk + o, my_s[b] + my_s[bm]);
+        atomicAdd(P.sumw + o, WEIGHTED ? my_w[b] + my_w[bm] : (double)c);
+      }
+    }
+    __syncthreads();
+    for (int b = tid; b < nb; b += blockDim.x) {
+      hc_cta[b] = 0ull;
+      my_s[b] = 0.0;
+      if constexpr (WEIGHTED) my_w[b] = 0.0;
+    }
+  };
 
   const double M = P.hi, lo2 = P.lo2;
-  const int4* slist = pb_super_list(P);
   const double* sup0 = pb_super_records(P);
-  const unsigned long long nlist = *P.slist_len;
-  unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0;   // leaf blocks, super pairs
-  int cur_cat = -1, since_flush = 0;
-  while (true) {
-    unsigned long long q = 0;
-    if (lane == 0) q = atomicAdd(P.counter, 1ull);
-    q = __shfl_sync(0xffffffffu, q, 0);
-    if (q >= nlist) break;
-    const int4 e = slist[q];
+  unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0, st_rows = 0;
+
+  // ---- one super pair (one warp) ----
+  auto decide = [&](const int4 e) {
     const int cat = e.x, wx0 = e.w & 0xffff, wy0 = e.w >> 16;
-    // <= 2^16 pairs per super pair and 2^31 / 2^16 super pairs per flush keep the 32-bit warp histogram counts exact
-    if (cat != cur_cat || since_flush >= (1 << 14)) {
-      flush_hist(cur_cat);
-      cur_cat = cat;
-      since_flush = 0;
-    }
-    ++since_flush;
     ++st_pairs;
     const int64_t off = P.cat_off[cat];
     const int64_t r0 = (int64_t)e.y * PB_SUPER, c0 = (int64_t)e.z * PB_SUPER;   // first row / column chunk
     const double* rec0 = P.boxes + (size_t)PB_STRIDE * (size_t)(off / PB_CHUNK + cat);
-    // The bit of each axis, fixed per super pair from the super-chunk boxes {xmin, xmax, ymin, ymax} (as
-    // pb_super_status decides): bin edge t = ed[x0 + 1] (bit 0 -> bin x0, bit 1 -> bin x0 + 1); upper range edge
-    // t = max_sep (bit 0 -> bin nbins - 1, bit 1 -> out of range); lower range edge t = the smallest double above
-    // -max_sep (bit 0 -> out, bit 1 -> bin 0).  The mirrored entry's upper bit is d <= m: m = -ed[nbins-1-x0] for a
-    // bin edge; for a range edge m = the double below t, so the mirror check passes by construction (the range test
-    // is the same for both entries, fl(x_i - x_j) = -fl(x_j - x_i), and the in-range mirrored window is the mirror
-    // image).
     const double4 rsb = *reinterpret_cast<const double4*>(sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat + e.y));
     const double4 csb = *reinterpret_cast<const double4*>(sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat + e.z));
-    const bool upx = csb.y - rsb.x >= M, lox = csb.x - rsb.y <= -M;
-    const bool upy = csb.w - rsb.z >= M, loy = csb.z - rsb.w <= -M;
-    const double tx = upx ? M : (lox ? nextafter(-M, 0.0) : ed[wx0 + 1]);
-    const double ty = upy ? M : (loy ? nextafter(-M, 0.0) : ed[wy0 + 1]);
-    const double mx = upx ? nextafter(M, 0.0) : (lox ? -M : -ed[nbins - 1 - wx0]);
-    const double my = upy ? nextafter(M, 0.0) : (loy ? -M : -ed[nbins - 1 - wy0]);
-    // forward bin of each bit value, -1 = out of range (dropped at booking)
-    const int bx0 = upx ? nbins - 1 : (lox ? -1 : wx0), bx1 = upx ? -1 : (lox ? 0 : wx0 + 1);
-    const int by0 = upy ? nbins - 1 : (loy ? -1 : wy0), by1 = upy ? -1 : (loy ? 0 : wy0 + 1);
+    const PBLeafBits B = pb_leaf_bits(rsb, csb, M, nbins, ed, wx0, wy0);
+    const double tx = B.tx, ty = B.ty, mx = B.mx, my = B.my;
     // the four forward bins of the super pair, per lane: all pairs, x-bit, y-bit, both bits
     unsigned n_t = 0u, n_x = 0u, n_y = 0u, n_xy = 0u;
     double s_t = 0.0, s_x = 0.0, s_y = 0.0, s_xy = 0.0, w_t = 0.0, w_x = 0.0, w_y = 0.0, w_xy = 0.0;
 
     // ---- classify the 64 leaf blocks: lane l takes column chunk l % 8 against row chunks l / 8 and l / 8 + 4 ----
+    // BOOK: closed blocks into the four sums (the per-block body); otherwise only the form class is kept
     const double* crec = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + (lane & 7));
-    const double4 cb = *reinterpret_cast<const double4*>(crec);
-    const double2 cs = *reinterpret_cast<const double2*>(crec + 4);
+    double2 cs = make_double2(0.0, 0.0);
     int code[2];
+    auto classify = [&](bool book) {
+      const double4 cb = *reinterpret_cast<const double4*>(crec);
+      cs = *reinterpret_cast<const double2*>(crec + 4);
 #pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const double* rrec = rec0 + (size_t)PB_STRIDE * (size_t)(r0 + (lane >> 3) + 4 * h);
-      const double4 rb = *reinterpret_cast<const double4*>(rrec);
-      int win[4];
-      const int cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, cb.x, cb.y, cb.z, cb.w, M, lo2, nbins, ed, win);
-      // per axis: 0 / 1 = the bit is constant, 2 = it varies (bin edge with a clean mirrored window, or the range edge
-      // runs through the block), 3 = neither (unclean mirrored window)
-      auto axis = [&](bool up, bool lo, double d0, double d1, int w, int rw, int a) -> int {
-        if (up || lo) return (up ? d1 >= M : d0 <= -M) ? 2 : (up ? 0 : 1);
-        const int x0 = w & 0xffff, rx0 = rw & 0xffff;
-        if ((w >> 16) == 0 && (rw >> 16) == 0 && rx0 == nbins - 1 - x0) return x0 - a;
-        if ((w >> 16) == 1 && (rw >> 16) == 1 && rx0 == nbins - 2 - x0) return 2;
-        return 3;
-      };
-      int bx = 3, by = 3;
-      if (cls == PB_REG_FULL || cls == PB_REG_CHECK) {
-        bx = axis(upx, lox, cb.x - rb.y, cb.y - rb.x, win[0], win[2], wx0);
-        by = axis(upy, loy, cb.z - rb.w, cb.w - rb.z, win[1], win[3], wy0);
-      }
-      int c = PB_L_OUT;
-      if (cls != PB_OUT) {
-        if (bx < 2 && by < 2) {   // every pair in range, in one slot
-          const double2 rs = *reinterpret_cast<const double2*>(rrec + 4);
-          const double s = rs.x * cs.x, w = WEIGHTED ? rs.y * cs.y : 0.0;
-          const unsigned n = (unsigned)(PB_CHUNK * PB_CHUNK);
-          n_t += n; s_t += s; w_t += w;
-          if (bx) { n_x += n; s_x += s; w_x += w; }
-          if (by) { n_y += n; s_y += s; w_y += w; }
-          if (bx && by) { n_xy += n; s_xy += s; w_xy += w; }
-          ++st_closed;
-        } else if (bx == 2 && by < 2) c = PB_L_ONE_X | (by << 3);   // x varies, the y bit is constant
-        else if (by == 2 && bx < 2) c = PB_L_ONE_Y | (bx << 3);
-        else c = (bx == 2 && by == 2 && (P.fast_paths & 2)) ? PB_L_QUAD : PB_L_PAIRS;
-        if (cls != PB_REG_FULL && c != PB_L_OUT) c |= 16;   // the range edge runs through the block
-      }
-      code[h] = c;
-    }
-    const unsigned act0 = __ballot_sync(0xffffffffu, code[0] != PB_L_OUT);
-    const unsigned act1 = __ballot_sync(0xffffffffu, code[1] != PB_L_OUT);
-
-    // ---- the other leaf blocks, one row chunk at a time: lane = row point ----
-    int staged = -1;   // column chunk staged in cxy / ck / cw
-    auto stage = [&](int c) {
-      if (c == staged) return;
-      const int64_t j = off + (c0 + c) * PB_CHUNK + lane;
-      double wj = 1.0;
-      if constexpr (WEIGHTED) wj = P.pw[j];
-      __syncwarp();
-      cxy[lane] = make_double2(P.px[j], P.py[j]);
-      ck[lane] = P.pk[j] * wj;
-      if constexpr (WEIGHTED) cw[lane] = wj;
-      __syncwarp();
-      staged = c;
-    };
-#pragma unroll 1
-    for (int rk = 0; rk < PB_SUPER; ++rk) {
-      unsigned m = ((rk < 4 ? act0 : act1) >> ((rk & 3) * 8)) & 0xffu;
-      if (!m) continue;
-      const int codes = rk < 4 ? code[0] : code[1];
-      const int64_t i = off + (r0 + rk) * PB_CHUNK + lane;
-      const double xi = P.px[i], yi = P.py[i];
-      double wi = 1.0;
-      if constexpr (WEIGHTED) wi = P.pw[i];
-      const double ki = P.pk[i] * wi;
-      // a block's column sums of k_j w_j (w_j) over all pairs, the x-bit, the y-bit and both bits, times this row
-      // point's k_i w_i (w_i)
-      auto book = [&](double at, double ax, double ay, double axy, double bt, double bx, double by, double bxy) {
-        s_t = fma(ki, at, s_t); s_x = fma(ki, ax, s_x); s_y = fma(ki, ay, s_y); s_xy = fma(ki, axy, s_xy);
-        if constexpr (WEIGHTED) {
-          w_t = fma(wi, bt, w_t); w_x = fma(wi, bx, w_x); w_y = fma(wi, by, w_y); w_xy = fma(wi, bxy, w_xy);
+      for (int h = 0; h < 2; ++h) {
+        const double* rrec = rec0 + (size_t)PB_STRIDE * (size_t)(r0 + (lane >> 3) + 4 * h);
+        const double4 rb = *reinterpret_cast<const double4*>(rrec);
+        int win[4];
+        const int cls = pb_classify_twod<true>(rb.x, rb.y, rb.z, rb.w, cb.x, cb.y, cb.z, cb.w, M, lo2, nbins, ed, win);
+        // per axis: 0 / 1 = the bit is constant, 2 = it varies (bin edge with a clean mirrored window, or the range
+        // edge runs through the block), 3 = neither (unclean mirrored window)
+        auto axis = [&](bool up, bool lo, double d0, double d1, int w, int rw, int a) -> int {
+          if (up || lo) return (up ? d1 >= M : d0 <= -M) ? 2 : (up ? 0 : 1);
+          const int x0 = w & 0xffff, rx0 = rw & 0xffff;
+          if ((w >> 16) == 0 && (rw >> 16) == 0 && rx0 == nbins - 1 - x0) return x0 - a;
+          if ((w >> 16) == 1 && (rw >> 16) == 1 && rx0 == nbins - 2 - x0) return 2;
+          return 3;
+        };
+        int bx = 3, by = 3;
+        if (cls == PB_REG_FULL || cls == PB_REG_CHECK) {
+          bx = axis(B.upx, B.lox, cb.x - rb.y, cb.y - rb.x, win[0], win[2], wx0);
+          by = axis(B.upy, B.loy, cb.z - rb.w, cb.w - rb.z, win[1], win[3], wy0);
         }
-      };
-      while (m) {
-        const int c = __ffs(m) - 1;
-        m &= m - 1;
-        const int lc = __shfl_sync(0xffffffffu, codes, (rk & 3) * 8 + c);
-        const int cls = lc & 7, cbit = (lc >> 3) & 1;
-        const bool check = (lc >> 4) & 1;
-        const double csk = __shfl_sync(0xffffffffu, cs.x, c);
-        double csw = 0.0;
-        if constexpr (WEIGHTED) csw = __shfl_sync(0xffffffffu, cs.y, c);
-        const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + c) + PB_SLOT;   // sorted copies of the chunk
-        bool per_pair = cls == PB_L_PAIRS;
-        if (cls == PB_L_ONE_X || cls == PB_L_ONE_Y) {
-          const bool vx = cls == PB_L_ONE_X;
-          const double* xs = vx ? srt : srt + 3 * PB_CHUNK;
-          int pos;
-          const bool ok = pb_rank_query_d(xs, vx ? xi : yi, vx ? tx : ty, vx ? mx : my, pos);
-          if (__all_sync(0xffffffffu, ok)) {
-            const unsigned bc = (unsigned)(PB_CHUNK - pos);
-            const double bs = pos < PB_CHUNK ? xs[PB_CHUNK + pos] : 0.0;
-            double bw = 0.0;
-            if constexpr (WEIGHTED) bw = pos < PB_CHUNK ? xs[2 * PB_CHUNK + pos] : 0.0;
-            // the varying axis' bit: the rank query; the constant axis' bit: cbit for every pair
-            const unsigned cc = cbit ? (unsigned)PB_CHUNK : 0u;
-            const double ck_ = cbit ? csk : 0.0, cw_ = cbit ? csw : 0.0;
-            n_t += PB_CHUNK;
-            n_x += vx ? bc : cc;
-            n_y += vx ? cc : bc;
-            n_xy += cbit ? bc : 0u;
-            book(csk, vx ? bs : ck_, vx ? ck_ : bs, cbit ? bs : 0.0, csw, vx ? bw : cw_, vx ? cw_ : bw, cbit ? bw : 0.0);
-            ++st_sorted;
-            continue;
-          }
-          ++st_1d;   // (rare) a column within rounding of a bin edge: pair by pair
-          per_pair = true;
-        } else if (cls == PB_L_QUAD) {
-          stage(c);
-          double qs = 0.0, qw = 0.0;
-          unsigned qc = 0u;
-#pragma unroll 4
-          for (int jj = 0; jj < PB_CHUNK; ++jj) {
-            const double2 pj = cxy[jj];
-            const bool p = (pj.x - xi >= tx) && (pj.y - yi >= ty);
-            const double mk = p ? 1.0 : 0.0;
-            qs = fma(ck[jj], mk, qs);
-            if constexpr (WEIGHTED) qw = fma(cw[jj], mk, qw);
-            qc += p ? 1u : 0u;
-          }
-          int posx, posy;
-          const bool okx = pb_rank_query_d(srt, xi, tx, mx, posx);
-          const bool oky = pb_rank_query_d(srt + 3 * PB_CHUNK, yi, ty, my, posy);
-          if (__all_sync(0xffffffffu, okx && oky)) {
-            n_t += PB_CHUNK;
-            n_x += (unsigned)(PB_CHUNK - posx);
-            n_y += (unsigned)(PB_CHUNK - posy);
-            n_xy += qc;
-            double bx = 0.0, by = 0.0;
-            if constexpr (WEIGHTED) {
-              bx = posx < PB_CHUNK ? srt[2 * PB_CHUNK + posx] : 0.0;
-              by = posy < PB_CHUNK ? srt[5 * PB_CHUNK + posy] : 0.0;
+        int c = PB_L_OUT;
+        if (cls != PB_OUT) {
+          if (bx < 2 && by < 2) {   // every pair in range, in one slot
+            if (book) {
+              const double2 rs = *reinterpret_cast<const double2*>(rrec + 4);
+              const double s = rs.x * cs.x, w = WEIGHTED ? rs.y * cs.y : 0.0;
+              const unsigned n = (unsigned)(PB_CHUNK * PB_CHUNK);
+              n_t += n; s_t += s; w_t += w;
+              if (bx) { n_x += n; s_x += s; w_x += w; }
+              if (by) { n_y += n; s_y += s; w_y += w; }
+              if (bx && by) { n_xy += n; s_xy += s; w_xy += w; }
             }
-            book(csk, posx < PB_CHUNK ? srt[PB_CHUNK + posx] : 0.0, posy < PB_CHUNK ? srt[4 * PB_CHUNK + posy] : 0.0, qs,
-                 csw, bx, by, qw);
-            ++st_quad;
-            continue;
+            ++st_closed;
+          } else if (bx == 2 && by < 2) c = PB_L_ONE_X | (by << 3);   // x varies, the y bit is constant
+          else if (by == 2 && bx < 2) c = PB_L_ONE_Y | (bx << 3);
+          else c = (bx == 2 && by == 2 && (P.fast_paths & 2)) ? PB_L_QUAD : PB_L_PAIRS;
+          if (cls != PB_REG_FULL && c != PB_L_OUT) c |= 16;   // the range edge runs through the block
+        }
+        code[h] = c;
+      }
+    };
+
+    // ---- the leaf blocks that are not closed, one row chunk at a time: lane = row point ----
+    auto per_block = [&]() {
+      const unsigned act0 = __ballot_sync(0xffffffffu, code[0] != PB_L_OUT);
+      const unsigned act1 = __ballot_sync(0xffffffffu, code[1] != PB_L_OUT);
+      int staged = -1;   // column chunk staged in cxy / ck / cw
+      auto stage = [&](int c) {
+        if (c == staged) return;
+        const int64_t j = off + (c0 + c) * PB_CHUNK + lane;
+        double wj = 1.0;
+        if constexpr (WEIGHTED) wj = P.pw[j];
+        __syncwarp();
+        cxy[lane] = make_double2(P.px[j], P.py[j]);
+        ck[lane] = P.pk[j] * wj;
+        if constexpr (WEIGHTED) cw[lane] = wj;
+        __syncwarp();
+        staged = c;
+      };
+#pragma unroll 1
+      for (int rk = 0; rk < PB_SUPER; ++rk) {
+        unsigned m = ((rk < 4 ? act0 : act1) >> ((rk & 3) * 8)) & 0xffu;
+        if (!m) continue;
+        const int codes = rk < 4 ? code[0] : code[1];
+        const int64_t i = off + (r0 + rk) * PB_CHUNK + lane;
+        const double xi = P.px[i], yi = P.py[i];
+        double wi = 1.0;
+        if constexpr (WEIGHTED) wi = P.pw[i];
+        const double ki = P.pk[i] * wi;
+        // a block's column sums of k_j w_j (w_j) over all pairs, the x-bit, the y-bit and both bits, times this row
+        // point's k_i w_i (w_i)
+        auto book = [&](double at, double ax, double ay, double axy, double bt, double bx, double by, double bxy) {
+          s_t = fma(ki, at, s_t); s_x = fma(ki, ax, s_x); s_y = fma(ki, ay, s_y); s_xy = fma(ki, axy, s_xy);
+          if constexpr (WEIGHTED) {
+            w_t = fma(wi, bt, w_t); w_x = fma(wi, bx, w_x); w_y = fma(wi, by, w_y); w_xy = fma(wi, bxy, w_xy);
           }
-          per_pair = true;
-        }
-        if (!per_pair) continue;
-        // pair by pair over the raw points of the chunk: every in-range pair sits in the window; blocks the range edge
-        // runs through test the range per pair (r2 >= lo2 holds for every pair of a TWO_AXIS super pair)
-        if (cls != PB_L_ONE_X && cls != PB_L_ONE_Y) ++st_pw;
-        stage(c);
-        unsigned mmc = 0u;
-        double a_t = 0.0, a_x = 0.0, a_y = 0.0, a_xy = 0.0, b_t = 0.0, b_x = 0.0, b_y = 0.0, b_xy = 0.0;
+        };
+        while (m) {
+          const int c = __ffs(m) - 1;
+          m &= m - 1;
+          const int lc = __shfl_sync(0xffffffffu, codes, (rk & 3) * 8 + c);
+          const int cls = lc & 7, cbit = (lc >> 3) & 1;
+          const bool check = (lc >> 4) & 1;
+          const double csk = __shfl_sync(0xffffffffu, cs.x, c);
+          double csw = 0.0;
+          if constexpr (WEIGHTED) csw = __shfl_sync(0xffffffffu, cs.y, c);
+          const double* srt = rec0 + (size_t)PB_STRIDE * (size_t)(c0 + c) + PB_SLOT;   // sorted copies of the chunk
+          bool per_pair = cls == PB_L_PAIRS;
+          if (cls == PB_L_ONE_X || cls == PB_L_ONE_Y) {
+            const bool vx = cls == PB_L_ONE_X;
+            const double* xs = vx ? srt : srt + 3 * PB_CHUNK;
+            int pos;
+            const bool ok = pb_rank_query_d(xs, vx ? xi : yi, vx ? tx : ty, vx ? mx : my, pos);
+            if (__all_sync(0xffffffffu, ok)) {
+              const unsigned bc = (unsigned)(PB_CHUNK - pos);
+              const double bs = pos < PB_CHUNK ? xs[PB_CHUNK + pos] : 0.0;
+              double bw = 0.0;
+              if constexpr (WEIGHTED) bw = pos < PB_CHUNK ? xs[2 * PB_CHUNK + pos] : 0.0;
+              // the varying axis' bit: the rank query; the constant axis' bit: cbit for every pair
+              const unsigned cc = cbit ? (unsigned)PB_CHUNK : 0u;
+              const double ck_ = cbit ? csk : 0.0, cw_ = cbit ? csw : 0.0;
+              n_t += PB_CHUNK;
+              n_x += vx ? bc : cc;
+              n_y += vx ? cc : bc;
+              n_xy += cbit ? bc : 0u;
+              book(csk, vx ? bs : ck_, vx ? ck_ : bs, cbit ? bs : 0.0, csw, vx ? bw : cw_, vx ? cw_ : bw, cbit ? bw : 0.0);
+              ++st_sorted;
+              continue;
+            }
+            ++st_1d;   // (rare) a column within rounding of a bin edge: pair by pair
+            per_pair = true;
+          } else if (cls == PB_L_QUAD) {
+            stage(c);
+            double qs = 0.0, qw = 0.0;
+            unsigned qc = 0u;
+#pragma unroll 4
+            for (int jj = 0; jj < PB_CHUNK; ++jj) {
+              const double2 pj = cxy[jj];
+              const bool p = (pj.x - xi >= tx) && (pj.y - yi >= ty);
+              const double mk = p ? 1.0 : 0.0;
+              qs = fma(ck[jj], mk, qs);
+              if constexpr (WEIGHTED) qw = fma(cw[jj], mk, qw);
+              qc += p ? 1u : 0u;
+            }
+            int posx, posy;
+            const bool okx = pb_rank_query_d(srt, xi, tx, mx, posx);
+            const bool oky = pb_rank_query_d(srt + 3 * PB_CHUNK, yi, ty, my, posy);
+            if (__all_sync(0xffffffffu, okx && oky)) {
+              n_t += PB_CHUNK;
+              n_x += (unsigned)(PB_CHUNK - posx);
+              n_y += (unsigned)(PB_CHUNK - posy);
+              n_xy += qc;
+              double bx = 0.0, by = 0.0;
+              if constexpr (WEIGHTED) {
+                bx = posx < PB_CHUNK ? srt[2 * PB_CHUNK + posx] : 0.0;
+                by = posy < PB_CHUNK ? srt[5 * PB_CHUNK + posy] : 0.0;
+              }
+              book(csk, posx < PB_CHUNK ? srt[PB_CHUNK + posx] : 0.0, posy < PB_CHUNK ? srt[4 * PB_CHUNK + posy] : 0.0,
+                   qs, csw, bx, by, qw);
+              ++st_quad;
+              continue;
+            }
+            per_pair = true;
+          }
+          if (!per_pair) continue;
+          // pair by pair over the raw points of the chunk: every in-range pair sits in the window; blocks the range
+          // edge runs through test the range per pair (r2 >= lo2 holds for every pair of a TWO_AXIS super pair)
+          if (cls != PB_L_ONE_X && cls != PB_L_ONE_Y) ++st_pw;
+          stage(c);
+          unsigned mmc = 0u;
+          double a_t = 0.0, a_x = 0.0, a_y = 0.0, a_xy = 0.0, b_t = 0.0, b_x = 0.0, b_y = 0.0, b_xy = 0.0;
 #pragma unroll 2
-        for (int jj = 0; jj < PB_CHUNK; ++jj) {
-          const double2 pj = cxy[jj];
-          const double dx = pj.x - xi, dy = pj.y - yi;
-          if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
-          const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
-          const double kj = ck[jj];
-          double wj = 0.0;
-          if constexpr (WEIGHTED) wj = cw[jj];
-          const double fx = px ? 1.0 : 0.0, fy = py ? 1.0 : 0.0, fxy = (px && py) ? 1.0 : 0.0;
-          n_t += 1u; n_x += px ? 1u : 0u; n_y += py ? 1u : 0u; n_xy += (px && py) ? 1u : 0u;
-          a_t += kj; a_x = fma(kj, fx, a_x); a_y = fma(kj, fy, a_y); a_xy = fma(kj, fxy, a_xy);
-          if constexpr (WEIGHTED) { b_t += wj; b_x = fma(wj, fx, b_x); b_y = fma(wj, fy, b_y); b_xy = fma(wj, fxy, b_xy); }
-          mmc += ((px != qx) && (py != qy)) ? 0u : 1u;
-        }
-        book(a_t, a_x, a_y, a_xy, b_t, b_x, b_y, b_xy);
-        if (__any_sync(0xffffffffu, mmc != 0u) && mmc) {
-          // (rare) pairs whose exact mirrored bin is not the mirror image of the forward bin: -1 at the assumed bin,
-          // +1 at the exact one, directly in global memory
-          const size_t g = (size_t)cat * nb;
           for (int jj = 0; jj < PB_CHUNK; ++jj) {
             const double2 pj = cxy[jj];
             const double dx = pj.x - xi, dy = pj.y - yi;
             if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
             const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
-            if ((px != qx) && (py != qy)) continue;
-            // only bin-edge bits can disagree; a range bit's mirrored bin is the mirror image
-            const int fx = px ? bx1 : bx0, fy = py ? by1 : by0;
-            const int ex = px != qx ? nbins - 1 - fx : nbins - 2 - wx0 + (qx ? 1 : 0);
-            const int ey = py != qy ? nbins - 1 - fy : nbins - 2 - wy0 + (qy ? 1 : 0);
-            const int assumed = (nbins - 1 - fy) * nbins + (nbins - 1 - fx), exact = ey * nbins + ex;
-            const double kk = ki * ck[jj];
-            double ww = 1.0;
-            if constexpr (WEIGHTED) ww = wi * cw[jj];
-            atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + assumed, ~0ull);   // -1 (mod 2^64)
-            atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + exact, 1ull);
-            atomicAdd(P.sumwkk + g + assumed, -kk);
-            atomicAdd(P.sumwkk + g + exact, kk);
-            atomicAdd(P.sumw + g + assumed, -ww);
-            atomicAdd(P.sumw + g + exact, ww);
+            const double kj = ck[jj];
+            double wj = 0.0;
+            if constexpr (WEIGHTED) wj = cw[jj];
+            const double fx = px ? 1.0 : 0.0, fy = py ? 1.0 : 0.0, fxy = (px && py) ? 1.0 : 0.0;
+            n_t += 1u; n_x += px ? 1u : 0u; n_y += py ? 1u : 0u; n_xy += (px && py) ? 1u : 0u;
+            a_t += kj; a_x = fma(kj, fx, a_x); a_y = fma(kj, fy, a_y); a_xy = fma(kj, fxy, a_xy);
+            if constexpr (WEIGHTED) { b_t += wj; b_x = fma(wj, fx, b_x); b_y = fma(wj, fy, b_y); b_xy = fma(wj, fxy, b_xy); }
+            mmc += ((px != qx) && (py != qy)) ? 0u : 1u;
+          }
+          book(a_t, a_x, a_y, a_xy, b_t, b_x, b_y, b_xy);
+          if (__any_sync(0xffffffffu, mmc != 0u) && mmc) {
+            // (rare) pairs whose exact mirrored bin is not the mirror image of the forward bin: -1 at the assumed
+            // bin, +1 at the exact one, directly in global memory
+            const size_t g = (size_t)cat * nb;
+            for (int jj = 0; jj < PB_CHUNK; ++jj) {
+              const double2 pj = cxy[jj];
+              const double dx = pj.x - xi, dy = pj.y - yi;
+              if (check && !(fabs(dx) < M && fabs(dy) < M)) continue;
+              const bool px = dx >= tx, py = dy >= ty, qx = dx <= mx, qy = dy <= my;
+              if ((px != qx) && (py != qy)) continue;
+              // only bin-edge bits can disagree; a range bit's mirrored bin is the mirror image
+              const int fx = px ? B.bx1 : B.bx0, fy = py ? B.by1 : B.by0;
+              const int ex = px != qx ? nbins - 1 - fx : nbins - 2 - wx0 + (qx ? 1 : 0);
+              const int ey = py != qy ? nbins - 1 - fy : nbins - 2 - wy0 + (qy ? 1 : 0);
+              const int assumed = (nbins - 1 - fy) * nbins + (nbins - 1 - fx), exact = ey * nbins + ex;
+              const double kk = ki * ck[jj];
+              double ww = 1.0;
+              if constexpr (WEIGHTED) ww = wi * cw[jj];
+              atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + assumed, ~0ull);   // -1 (mod 2^64)
+              atomicAdd(reinterpret_cast<unsigned long long*>(P.npairs) + g + exact, 1ull);
+              atomicAdd(P.sumwkk + g + assumed, -kk);
+              atomicAdd(P.sumwkk + g + exact, kk);
+              atomicAdd(P.sumw + g + assumed, -ww);
+              atomicAdd(P.sumw + g + exact, ww);
+            }
           }
         }
       }
+    };
+
+    bool rows_ok = false;
+    if constexpr (STAGED) {
+      // ---- per row point against the staged column super-chunk: p_x, p_y by bisection, the quadrant from the table
+      const int SP = PB_SUPER_PTS, XB = PB_LT_XB, N = PB_LT_N;
+      const int64_t rb = off + (int64_t)e.y * PB_SUPER_PTS + lane;
+      const double csk = T.sxk[0];
+      double csw = 0.0;
+      if constexpr (WEIGHTED) csw = T.sxw[0];
+      bool ok = true;
+#pragma unroll 2
+      for (int k = 0; k < PB_SUPER; ++k) {
+        const int64_t i = rb + k * 32;
+        const double xi = P.px[i], yi = P.py[i];
+        double wi = 1.0;
+        if constexpr (WEIGHTED) wi = P.pw[i];
+        const double ki = P.pk[i] * wi;
+        int px = 0, py = 0;   // #{j : fl(c_j - c_i) < t} (branch-free lower bounds over the ascending copies)
+#pragma unroll
+        for (int step = SP / 2; step >= 1; step >>= 1) {
+          if (T.xs[px + step - 1] - xi < tx) px += step;
+          if (T.ys[py + step - 1] - yi < ty) py += step;
+        }
+        if (px == SP - 1 && T.xs[px] - xi < tx) px = SP;
+        if (py == SP - 1 && T.ys[py] - yi < ty) py = SP;
+        // exact mirrored bits: consistent iff the column below each split has the mirrored upper bit and the column at
+        // the split has not
+        ok = ok && (px == 0 || T.xs[px - 1] - xi <= mx) && (px == SP || !(T.xs[px] - xi <= mx)) &&
+             (py == 0 || T.ys[py - 1] - yi <= my) && (py == SP || !(T.ys[py] - yi <= my));
+        const int b = min(px / XB, PB_LT_NB - 1), xo = px % XB;
+        const int q = T.qr[b * N + py];
+        unsigned qc = T.uc[(b + 1) * N + py] + __popc(T.msk[b * (XB + 1) + q] >> xo);
+        double qs = T.uk[(b + 1) * N + py] + T.vk[(b * XB + xo) * (XB + 1) + q];
+        if (px == SP) { qc = 0u; qs = 0.0; }
+        n_t += (unsigned)SP;
+        n_x += (unsigned)(SP - px);
+        n_y += (unsigned)(SP - py);
+        n_xy += qc;
+        s_t = fma(ki, csk, s_t);
+        s_x = fma(ki, T.sxk[px], s_x);
+        s_y = fma(ki, T.syk[py], s_y);
+        s_xy = fma(ki, qs, s_xy);
+        if constexpr (WEIGHTED) {
+          double qw = T.uw[(b + 1) * N + py] + T.vw[(b * XB + xo) * (XB + 1) + q];
+          if (px == SP) qw = 0.0;
+          w_t = fma(wi, csw, w_t);
+          w_x = fma(wi, T.sxw[px], w_x);
+          w_y = fma(wi, T.syw[py], w_y);
+          w_xy = fma(wi, qw, w_xy);
+        }
+      }
+      rows_ok = __all_sync(0xffffffffu, ok);
+    }
+    if (rows_ok) {   // the leaf blocks only for the path statistics, by form class
+      classify(false);
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int cls = code[h] & 7;
+        st_sorted += __popc(__ballot_sync(0xffffffffu, cls == PB_L_ONE_X || cls == PB_L_ONE_Y));
+        st_quad += __popc(__ballot_sync(0xffffffffu, cls == PB_L_QUAD));
+        st_pw += __popc(__ballot_sync(0xffffffffu, cls == PB_L_PAIRS));
+      }
+      ++st_rows;
+    } else {
+      n_t = n_x = n_y = n_xy = 0u;
+      s_t = s_x = s_y = s_xy = w_t = w_x = w_y = w_xy = 0.0;
+      classify(true);
+      per_block();
     }
 
-    // ---- the four bins of the window into the warp histogram (forward entries) ----
+    // ---- the four bins of the window into the histogram (forward entries) ----
     n_t = warp_sum_u(n_t); n_x = warp_sum_u(n_x); n_y = warp_sum_u(n_y); n_xy = warp_sum_u(n_xy);
     s_t = warp_sum(s_t); s_x = warp_sum(s_x); s_y = warp_sum(s_y); s_xy = warp_sum(s_xy);
     if constexpr (WEIGHTED) { w_t = warp_sum(w_t); w_x = warp_sum(w_x); w_y = warp_sum(w_y); w_xy = warp_sum(w_xy); }
-    if (lane == 0) {   // inclusion-exclusion per slot (index = bx + 2 by), out-of-range slots dropped; private histogram
+    if (lane == 0) {   // inclusion-exclusion per slot (index = bx + 2 by), out-of-range slots dropped
       const unsigned fc[4] = {n_t - n_x - n_y + n_xy, n_x - n_xy, n_y - n_xy, n_xy};
       const double fs[4] = {(s_t - s_x) - (s_y - s_xy), s_x - s_xy, s_y - s_xy, s_xy};
       const double fw[4] = {(w_t - w_x) - (w_y - w_xy), w_x - w_xy, w_y - w_xy, w_xy};
 #pragma unroll
       for (int b = 0; b < 4; ++b) {
-        const int fx = (b & 1) ? bx1 : bx0, fy = (b >> 1) ? by1 : by0;
+        const int fx = (b & 1) ? B.bx1 : B.bx0, fy = (b >> 1) ? B.by1 : B.by0;
         if (fc[b] && fx >= 0 && fy >= 0) {
           const int o = fy * nbins + fx;
-          my_c[o] += fc[b];
-          my_s[o] += fs[b];
-          if constexpr (WEIGHTED) my_w[o] += fw[b];
+          if constexpr (STAGED) {   // the CTA histogram
+            atomicAdd(hc_cta + o, (unsigned long long)fc[b]);
+            atomicAdd(my_s + o, fs[b]);
+            if constexpr (WEIGHTED) atomicAdd(my_w + o, fw[b]);
+          } else {                  // the private warp histogram
+            my_c[o] += fc[b];
+            my_s[o] += fs[b];
+            if constexpr (WEIGHTED) my_w[o] += fw[b];
+          }
         }
       }
     }
     __syncwarp();
+  };
+
+  if constexpr (STAGED) {
+    __shared__ unsigned long long s_item;
+    __shared__ unsigned s_next;
+    const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
+    const unsigned long long nitems = P.slist_len[2];
+    const int nthr = blockDim.x, nwarps = nthr >> 5;
+    const int SP = PB_SUPER_PTS, XB = PB_LT_XB, N = PB_LT_N;
+    int cur_cat = -1;
+    while (true) {
+      __syncthreads();   // the previous item's tables are consumed
+      if (tid == 0) {
+        const unsigned long long q = atomicAdd(P.counter, 1ull);
+        s_item = q < nitems ? grp.items[q] : ~0ull;
+        s_next = 0u;
+      }
+      __syncthreads();
+      const unsigned long long item = s_item;
+      if (item == ~0ull) break;
+      const int4* slice = grp.glist + (item >> 16);
+      const int len = (int)(item & 0xffff);
+      const int4 e0 = slice[0];
+      if (e0.x != cur_cat) {
+        flush_cta(cur_cat);
+        cur_cat = e0.x;
+      }
+      // ---- stage column super-chunk C: sorted copies, suffix sums, k w and w in x order, the links ----
+      {
+        const int64_t off = P.cat_off[e0.x], slot = off / PB_SUPER_PTS + e0.x + e0.z;
+        const double* crec = sup0 + (size_t)PB_SUPER_STRIDE * (size_t)slot + PB_SLOT;
+        const unsigned short* lk = grp.links + (size_t)PB_SUPER_PTS * (size_t)slot;
+        const int64_t base = off + (int64_t)e0.z * PB_SUPER_PTS;
+        for (int i = tid; i < SP; i += nthr) {
+          T.xs[i] = crec[i];
+          T.sxk[i] = crec[SP + i];
+          T.ys[i] = crec[3 * SP + i];
+          T.syk[i] = crec[4 * SP + i];
+          const unsigned l = lk[i];
+          const int j = (int)(l & 0xffu), r = (int)(l >> 8);
+          double wj = 1.0;
+          if constexpr (WEIGHTED) {
+            T.sxw[i] = crec[2 * SP + i];
+            T.syw[i] = crec[5 * SP + i];
+            wj = P.pw[base + j];
+            T.wx[i] = wj;
+          }
+          T.kx[i] = P.pk[base + j] * wj;
+          T.yr[i] = (unsigned char)r;
+          T.xp[r] = (unsigned char)i;
+        }
+        if (tid == 0) {
+          T.sxk[SP] = 0.0;
+          T.syk[SP] = 0.0;
+          if constexpr (WEIGHTED) { T.sxw[SP] = 0.0; T.syw[SP] = 0.0; }
+        }
+        for (int i = tid; i < N; i += nthr) {   // row NB of U: no x-block
+          T.uk[PB_LT_NB * N + i] = 0.0;
+          T.uc[PB_LT_NB * N + i] = 0;
+          if constexpr (WEIGHTED) T.uw[PB_LT_NB * N + i] = 0.0;
+        }
+      }
+      __syncthreads();
+      // in-block y order of every x position; U row by row (one warp per x-block: suffix scans over the y order)
+      for (int p = tid; p < SP; p += nthr) {
+        const int b0 = p & ~(XB - 1), r = T.yr[p];
+        int c = 0;
+#pragma unroll
+        for (int o = 0; o < XB; ++o) c += T.yr[b0 + o] < r ? 1 : 0;
+        T.yo[p] = (unsigned char)c;
+      }
+      for (int b = warp; b < PB_LT_NB; b += nwarps) {
+        double ak = 0.0, aw = 0.0;
+        unsigned ac = 0u;
+        for (int sg = SP / 32 - 1; sg >= 0; --sg) {
+          const int q = sg * 32 + lane, p = T.xp[q];
+          const bool in = p >= b * XB;
+          double vk = in ? T.kx[p] : 0.0, vw = 0.0;
+          if constexpr (WEIGHTED) vw = in ? T.wx[p] : 0.0;
+          unsigned vc = in ? 1u : 0u;
+#pragma unroll
+          for (int o = 1; o < 32; o <<= 1) {
+            const double tk = __shfl_down_sync(0xffffffffu, vk, o);
+            const unsigned tc = __shfl_down_sync(0xffffffffu, vc, o);
+            double tw = 0.0;
+            if constexpr (WEIGHTED) tw = __shfl_down_sync(0xffffffffu, vw, o);
+            if (lane + o < 32) { vk += tk; vc += tc; if constexpr (WEIGHTED) vw += tw; }
+          }
+          vk += ak; vc += ac;
+          T.uk[b * N + q] = vk;
+          T.uc[b * N + q] = (unsigned short)vc;
+          if constexpr (WEIGHTED) { vw += aw; T.uw[b * N + q] = vw; aw = __shfl_sync(0xffffffffu, vw, 0); }
+          ak = __shfl_sync(0xffffffffu, vk, 0);
+          ac = __shfl_sync(0xffffffffu, vc, 0);
+        }
+        if (lane == 0) {
+          T.uk[b * N + SP] = 0.0;
+          T.uc[b * N + SP] = 0;
+          if constexpr (WEIGHTED) T.uw[b * N + SP] = 0.0;
+        }
+      }
+      __syncthreads();
+      for (int i = tid; i < PB_LT_NB * N; i += nthr) T.qr[i] = (unsigned char)(XB - (T.uc[i] - T.uc[i + N]));
+      for (int i = tid; i < PB_LT_NB * (XB + 1); i += nthr) {   // V and the masks: suffix over the in-block x offset
+        const int b = i / (XB + 1), q = i % (XB + 1);
+        double ak = 0.0, aw = 0.0;
+        unsigned m = 0u;
+        for (int xo = XB - 1; xo >= 0; --xo) {
+          const int p = b * XB + xo;
+          if (T.yo[p] >= q) {
+            ak += T.kx[p];
+            if constexpr (WEIGHTED) aw += T.wx[p];
+            m |= 1u << xo;
+          }
+          T.vk[(b * XB + xo) * (XB + 1) + q] = ak;
+          if constexpr (WEIGHTED) T.vw[(b * XB + xo) * (XB + 1) + q] = aw;
+        }
+        T.msk[i] = m;
+      }
+      __syncthreads();
+      // ---- the slice's super pairs, one per warp step ----
+      while (true) {
+        unsigned k = 0;
+        if (lane == 0) k = atomicAdd(&s_next, 1u);
+        k = __shfl_sync(0xffffffffu, k, 0);
+        if ((int)k >= len) break;
+        decide(slice[k]);
+      }
+    }
+    flush_cta(cur_cat);
+  } else {
+    const int4* slist = pb_super_list(P);
+    const unsigned long long nlist = *P.slist_len;
+    int cur_cat = -1, since_flush = 0;
+    while (true) {
+      unsigned long long q = 0;
+      if (lane == 0) q = atomicAdd(P.counter, 1ull);
+      q = __shfl_sync(0xffffffffu, q, 0);
+      if (q >= nlist) break;
+      const int4 e = slist[q];
+      // <= 2^16 pairs per super pair and 2^31 / 2^16 super pairs per flush keep the 32-bit warp histogram counts exact
+      if (e.x != cur_cat || since_flush >= (1 << 14)) {
+        flush_hist(cur_cat);
+        cur_cat = e.x;
+        since_flush = 0;
+      }
+      ++since_flush;
+      decide(e);
+    }
+    flush_hist(cur_cat);
   }
-  flush_hist(cur_cat);
   const unsigned long long LEAF = (unsigned long long)PB_CHUNK * PB_CHUNK;
   if (st_closed) atomicAdd(&g_pb_stats[0], LEAF * st_closed);   // per classifying lane
   if (lane == 0) {
@@ -2329,6 +2768,7 @@ pairbin_super_leaves_kernel(PBParams P) {
     if (st_sorted) atomicAdd(&g_pb_stats[3], LEAF * st_sorted);
     if (st_quad) atomicAdd(&g_pb_stats[4], LEAF * st_quad);
     if (st_pairs) atomicAdd(&g_pb_super_leaves, (unsigned long long)st_pairs);
+    if (st_rows) atomicAdd(&g_pb_super_rows, (unsigned long long)st_rows);
   }
 }
 
@@ -2352,16 +2792,17 @@ static int64_t pb_rec_slots(int64_t max_len, int32_t ncat) {
   return ((int64_t)need + 255) / 256 * 256;
 }
 // Work buffer of the two-pass count: {work counters of pass A, pass B, the super kernel; length of the TWO_AXIS list,
-// work counter of the leaf kernel; 3 spare words} {record counts of a round: slots / 32 ints} {records: 2 doubles each}
-// {pre-pass chunk records} {super-chunk records} {TWO_AXIS list: 2 doubles per super pair}.  The other paths keep the
-// chunk records at the start.
+// work counter of the leaf kernel, its number of work items; 2 spare words} {record counts of a round: slots / 32 ints}
+// {records: 2 doubles each} {pre-pass chunk records} {super-chunk records} {TWO_AXIS list: 2 doubles per super pair}
+// {the regions of pb_super_groups}.  The other paths keep the chunk records at the start.
 static int64_t pb_rec_region_doubles(int64_t slots) { return 8 + slots / 64 + 2 * slots; }
 
 extern "C" int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat) {
-  const int64_t nsup = total_points / PB_SUPER_PTS;   // every catalogue's full super-chunks together
+  const int64_t nslot = pb_super_slots(total_points, ncat);
   return pb_rec_region_doubles(pb_rec_slots(total_points, ncat)) +
-         (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2) +
-         (int64_t)PB_SUPER_STRIDE * (nsup + (int64_t)ncat + 2) + nsup * (nsup > 0 ? nsup - 1 : 0);
+         (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2) + (int64_t)PB_SUPER_STRIDE * nslot +
+         4 * pb_super_list_cap(total_points) + (int64_t)PB_SUPER_PTS / 4 * nslot + ((nslot + 1) & ~(int64_t)1) +
+         pb_super_items_cap(total_points, ncat);
 }
 
 static int g_pb_fast_paths = 7;   // tgp_set_option("pairbin_fast_paths", bits): see PBParams::fast_paths
@@ -2375,6 +2816,16 @@ extern "C" int tgp_pairbin_super_leaves(unsigned long long* host1, int reset) {
   if (reset) {
     const unsigned long long z = 0;
     TGP_CUDA(cudaMemcpyToSymbol(g_pb_super_leaves, &z, sizeof(z)));
+  }
+  return TGP_OK;
+}
+
+extern "C" int tgp_pairbin_super_rows(unsigned long long* host1, int reset) {
+  TGP_CHECK_ARG(host1 != nullptr, "host1");
+  TGP_CUDA(cudaMemcpyFromSymbol(host1, g_pb_super_rows, sizeof(unsigned long long)));
+  if (reset) {
+    const unsigned long long z = 0;
+    TGP_CUDA(cudaMemcpyToSymbol(g_pb_super_rows, &z, sizeof(z)));
   }
   return TGP_OK;
 }
@@ -2490,7 +2941,7 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
 
   if (split) {
     // [0] pass A's work counter, [1] pass B's, [2] the super kernel's, [3] the TWO_AXIS list length, [4] the leaf
-    // kernel's work counter
+    // kernel's work counter, [5] its number of work items (staged; written by pairbin_super_group_kernel)
     unsigned long long* ctr = reinterpret_cast<unsigned long long*>(work);
     P.rec_cnt = reinterpret_cast<int*>(work + 8);
     P.recs = reinterpret_cast<int4*>(work + 8 + rec_slots / 64);
@@ -2532,28 +2983,61 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
       if (weighted) pairbin_super_kernel<true><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
       else pairbin_super_kernel<false><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
       TGP_LAUNCH_CHECK();
-      // the leaf kernel takes the TWO_AXIS super pairs the super kernel listed (the length stays on the device):
-      // warp histograms + one staged column chunk per warp; per_warp_l < per_warp_s, so warps_l >= 1
+      // the leaf kernel takes the TWO_AXIS super pairs the super kernel listed (the length stays on the device).
+      // Staged (the per-row form of the 2 x 2 window is on): the list grouped by column super-chunk, the tables of one
+      // super-chunk + a CTA histogram + one staged column chunk per warp, 2 CTAs of 8 warps per SM, or one of 16 if
+      // only that fits.  Otherwise warp histograms + one staged column chunk per warp; per_warp_l < per_warp_s, so
+      // warps_l >= 1.
       PBParams PL = P;
-      const size_t per_warp_l = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0)) + PB_CHUNK * (16 + 8 + 8);
-      int warps_l = (int)((budget - fixed - 64) / per_warp_l);
-      if (warps_l > PB_MAX_WARPS) warps_l = PB_MAX_WARPS;
-      PL.warps = warps_l;
       PL.counter = ctr + 4;
       PL.slist_len = ctr + 3;
-      const size_t smem_l = fixed + (size_t)warps_l * per_warp_l + 64;
-      int ctas_l = (int)((220 * 1024) / smem_l);
-      if (ctas_l > PB_LEAVES_MIN_CTAS) ctas_l = PB_LEAVES_MIN_CTAS;
-      if (ctas_l < 1) ctas_l = 1;
-      static TgpPerDeviceOnce once_l[2];
-      const void* kern_l = weighted ? (const void*)pairbin_super_leaves_kernel<true>
-                                    : (const void*)pairbin_super_leaves_kernel<false>;
-      if (tgp_first_use_on_device(once_l[weighted ? 1 : 0]))
-        TGP_CUDA(cudaFuncSetAttribute(kern_l, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
-      const unsigned grid_l = (unsigned)((int64_t)sms * ctas_l);
-      if (weighted) pairbin_super_leaves_kernel<true><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
-      else pairbin_super_leaves_kernel<false><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
-      TGP_LAUNCH_CHECK();
+      const size_t hist_t = (size_t)P.nb * (8 + 8 + (weighted ? 8 : 0));
+      auto smem_t = [&](int w) {
+        return fixed + (size_t)w * PB_CHUNK * (16 + 8 + 8) + hist_t + pb_leaf_table_bytes(weighted) + 64;
+      };
+      // what one CTA takes of the SM's 228 KB: dynamic + static shared memory (the item and pair claims) + the 1 KB the
+      // driver reserves per CTA, in 128-byte allocation units
+      auto cta_t = [&](int w) { return (smem_t(w) + 16 + 1024 + 127) / 128 * 128; };
+      int warps_t = 0, ctas_t = 0;
+      if (P.fast_paths & 2) {
+        if (2 * cta_t(PB_MAX_WARPS) <= 228 * 1024) { warps_t = PB_MAX_WARPS; ctas_t = 2; }
+        else if (smem_t(2 * PB_MAX_WARPS) <= 226 * 1024) { warps_t = 2 * PB_MAX_WARPS; ctas_t = 1; }
+      }
+      if (warps_t) {
+        pairbin_super_group_kernel<<<1, 1024, 0, st>>>(PL);
+        TGP_LAUNCH_CHECK();
+        pairbin_super_scatter_kernel<<<(unsigned)(sms * 4), 256, 0, st>>>(PL);
+        TGP_LAUNCH_CHECK();
+        PL.warps = warps_t;
+        const size_t smem_l = smem_t(warps_t);
+        static TgpPerDeviceOnce once_t[2];
+        const void* kern_t = weighted ? (const void*)pairbin_super_leaves_kernel<true, true>
+                                      : (const void*)pairbin_super_leaves_kernel<false, true>;
+        if (tgp_first_use_on_device(once_t[weighted ? 1 : 0]))
+          TGP_CUDA(cudaFuncSetAttribute(kern_t, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
+        const unsigned grid_t = (unsigned)((int64_t)sms * ctas_t);
+        if (weighted) pairbin_super_leaves_kernel<true, true><<<grid_t, warps_t * 32, smem_l, st>>>(PL);
+        else pairbin_super_leaves_kernel<false, true><<<grid_t, warps_t * 32, smem_l, st>>>(PL);
+        TGP_LAUNCH_CHECK();
+      } else {
+        const size_t per_warp_l = (size_t)P.nb * (8 + 4 + (weighted ? 8 : 0)) + PB_CHUNK * (16 + 8 + 8);
+        int warps_l = (int)((budget - fixed - 64) / per_warp_l);
+        if (warps_l > PB_MAX_WARPS) warps_l = PB_MAX_WARPS;
+        PL.warps = warps_l;
+        const size_t smem_l = fixed + (size_t)warps_l * per_warp_l + 64;
+        int ctas_l = (int)((220 * 1024) / smem_l);
+        if (ctas_l > PB_LEAVES_MIN_CTAS) ctas_l = PB_LEAVES_MIN_CTAS;
+        if (ctas_l < 1) ctas_l = 1;
+        static TgpPerDeviceOnce once_l[2];
+        const void* kern_l = weighted ? (const void*)pairbin_super_leaves_kernel<true, false>
+                                      : (const void*)pairbin_super_leaves_kernel<false, false>;
+        if (tgp_first_use_on_device(once_l[weighted ? 1 : 0]))
+          TGP_CUDA(cudaFuncSetAttribute(kern_l, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget));
+        const unsigned grid_l = (unsigned)((int64_t)sms * ctas_l);
+        if (weighted) pairbin_super_leaves_kernel<true, false><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
+        else pairbin_super_leaves_kernel<false, false><<<grid_l, warps_l * 32, smem_l, st>>>(PL);
+        TGP_LAUNCH_CHECK();
+      }
     }
     PBParams PA = P;
     PA.block_sums = supers ? 2 : 1;
