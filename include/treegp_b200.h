@@ -264,6 +264,22 @@ int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, con
 int tgp_predict_mean_batch(const double* Xs, const int64_t* soff /*host*/, const double* X, const int64_t* off /*host*/,
                            int32_t B, const tgp_kernel_sum* ks /*host*/, const double* alpha, double* mean,
                            void* stream);
+/* per-problem scratch of tgp_loglike_grad_batch: sum_b of the single gradient's scratch for N_b with
+ * 4 TGP_MAX_TERMS + 1 partial columns (tgp_loglike_grad_sum_work_doubles(N_b, TGP_MAX_TERMS)); problem b's block
+ * starts at the sum over c < b.  -1 for invalid B / off. */
+int64_t tgp_loglike_grad_batch_work_doubles(const int64_t* off /*host*/, int32_t B);
+/* tgp_loglike_grad_sum (dense, row_end == NULL) for every problem of a batch.  Arguments as tgp_loglike_batch, plus
+ * scratch (tgp_loglike_grad_batch_work_doubles doubles, 16-byte aligned).
+ * out: device double[B * TGP_GRAD_BATCH_OUT].  Problem b's slice has tgp_loglike_grad_sum's layout for ks[b]:
+ * {logL, chi2, logdet, 4 derivatives per term, d / d ln white} (one term without white: 4 derivatives, then 0).
+ * Unused tail entries are 0.  The gradient is 0 where info_b != 0.  On exit each problem's work block holds Z = K^-1
+ * (lower triangle, mirrored into the upper), equal to tgp_selinv on its factor bit for bit, and alpha = K^-1 y as with
+ * want_alpha != 0.  So logL, chi2 and logdet are tgp_loglike_batch's, and the gradient agrees with
+ * tgp_loglike_grad_sum on that problem alone to the rounding of alpha. */
+#define TGP_GRAD_BATCH_OUT (4 + 4 * TGP_MAX_TERMS)
+int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off /*host*/,
+                           int32_t B, const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, double* out,
+                           int32_t* info, double* scratch, void* stream);
 
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 

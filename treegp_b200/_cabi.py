@@ -26,6 +26,7 @@ class TgpKernel(ctypes.Structure):
 MAX_TERMS = 4   # TGP_MAX_TERMS
 MAX_RHS = 8     # TGP_MAX_RHS: outputs of the multi-output entries
 BATCH_MAX_N = 4096   # TGP_BATCH_MAX_N: points per problem of the batch entries
+GRAD_BATCH_OUT = 4 + 4 * MAX_TERMS   # TGP_GRAD_BATCH_OUT: outputs per problem of tgp_loglike_grad_batch
 
 
 class TgpKernelSum(ctypes.Structure):
@@ -79,6 +80,8 @@ SIGNATURES = {
     "tgp_batch_work_doubles": [_vp, _i32],
     "tgp_loglike_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, ctypes.c_int, _vp, _vp, _vp],
     "tgp_predict_mean_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
+    "tgp_loglike_grad_batch_work_doubles": [_vp, _i32],
+    "tgp_loglike_grad_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -115,6 +118,7 @@ _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctyp
              "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
              "tgp_loglike_grad_multi_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64, "tgp_batch_work_doubles": ctypes.c_int64,
+             "tgp_loglike_grad_batch_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 
 _lib = None

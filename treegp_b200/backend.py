@@ -374,13 +374,26 @@ def batch_work_doubles(sizes):
     return int(np.sum((n + 1) * ((n + 1) & ~1)))
 
 
-def plan_batch_chunks(sizes, budget_bytes):
-    """Split problems with `sizes` points, in order, into consecutive chunks whose loglike_batch workspace fits
-    `budget_bytes`; a problem larger than the budget gets a chunk of its own.  Pure host function: returns a list of
-    (start, stop) index pairs covering range(len(sizes))."""
+def grad_batch_scratch_doubles(sizes):
+    """Scratch of tgp_loglike_grad_batch: sum_b of tgp_loglike_grad_sum_work_doubles(N_b, TGP_MAX_TERMS), i.e. the
+    larger of the selected-inverse blocks (2 OB^2 + OB even(N)) and 4 TGP_MAX_TERMS + 1 partial sums per 64 x 64
+    contraction tile, plus even(ceil(N / OB)) for the envelope copy (OB = 512)."""
+    n = np.asarray(sizes, dtype=np.int64)
+    ob, ev = 512, (n + 1) & ~1
+    nt = (n + 63) // 64
+    selinv = 2 * ob * ob + ob * ev
+    partials = (4 * _cabi.MAX_TERMS + 1) * (nt * (nt + 1) // 2)
+    nblk = (n + ob - 1) // ob
+    return int(np.sum(np.maximum(selinv, partials) + ((nblk + 1) & ~1)))
+
+
+def plan_batch_chunks(sizes, budget_bytes, scratch=False):
+    """Split problems with `sizes` points, in order, into consecutive chunks whose loglike_batch workspace (plus, with
+    scratch=True, the loglike_grad_batch scratch) fits `budget_bytes`; a problem larger than the budget gets a chunk of
+    its own.  Pure host function: returns a list of (start, stop) index pairs covering range(len(sizes))."""
     chunks, start, used = [], 0, 0
     for b, n in enumerate(sizes):
-        need = 8 * batch_work_doubles([n])
+        need = 8 * batch_work_doubles([n]) + (8 * grad_batch_scratch_doubles([n]) if scratch else 0)
         if b > start and used + need > budget_bytes:
             chunks.append((start, b))
             start, used = b, 0
@@ -429,6 +442,33 @@ def loglike_batch(X, y, yerr2, sizes, descs, want_alpha=False, budget_bytes=4 <<
         check(lib.tgp_loglike_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
                                     ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]), int(bool(want_alpha)),
                                     _p(out[b0:b1]), _p(info[b0:b1]), _stream()), "tgp_loglike_batch")
+    return out, info, alpha
+
+
+def loglike_grad_batch(X, y, yerr2, sizes, descs, budget_bytes=4 << 30):
+    """tgp_loglike_grad_batch over B problems, arguments as loglike_batch: each problem's log-likelihood and its
+    gradient in one pass, in chunks whose workspace plus scratch fit `budget_bytes` (plan_batch_chunks(scratch=True));
+    the results do not depend on the chunking.  Returns (out (B, TGP_GRAD_BATCH_OUT): per problem the layout of
+    loglike_grad for a sum, {logL, chi2, logdet, 4 derivatives per term, d / d ln white}, zero-padded; info (B,);
+    alpha (sum N_b,) = K^-1 y)."""
+    X = as_points(X)
+    sizes = [int(n) for n in sizes]
+    _check_batch_inputs(X, sizes, descs)
+    off = batch_offsets(sizes)
+    B = len(sizes)
+    out = torch.empty((B, _cabi.GRAD_BATCH_OUT), dtype=F64, device=X.device)
+    info = torch.empty(B, dtype=torch.int32, device=X.device)
+    alpha = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    lib = _cabi.load()
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True):
+        r0, r1 = int(off[b0]), int(off[b1])
+        o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
+        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        scratch = torch.empty(grad_batch_scratch_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        ks = _ksum_array(descs[b0:b1])
+        check(lib.tgp_loglike_grad_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                         ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]), _p(out[b0:b1]),
+                                         _p(info[b0:b1]), _p(scratch), _stream()), "tgp_loglike_grad_batch")
     return out, info, alpha
 
 

@@ -1,5 +1,5 @@
-// Batches of independent small problems: B likelihood evaluations (tgp_loglike_batch) or B posterior means
-// (tgp_predict_mean_batch) per call.
+// Batches of independent small problems: B likelihood evaluations (tgp_loglike_batch), B likelihoods with their
+// gradients (tgp_loglike_grad_batch) or B posterior means (tgp_predict_mean_batch) per call.
 //
 // A problem of a few hundred to a few thousand points leaves the B200 idle: its factorisation is a chain of small
 // launches (8 panel launches and one update per 512 columns, at most ~70 CTAs each), so its time is launch latency.
@@ -7,7 +7,8 @@
 // problem, each CTA picks its problem from blockIdx.x and runs the body of the single-problem kernel on that
 // problem's slice (kmat.cu, dense.cu, predict.cu), and CTAs of problems without work at that step exit.  So a
 // problem's K, factor, logL and info are what tgp_loglike_sum (dense) gives on it alone, bit for bit, whatever else
-// shares the batch.  The only new arithmetic is the backward sweep of want_alpha (one CTA per problem, below).
+// shares the batch.  The only new arithmetic is the backward sweep of want_alpha (one CTA per problem, below).  The
+// gradient adds the selected inverse, contraction and finish of tgp_loglike_grad_sum in the same form (selinv.cu).
 #include <string.h>
 #include <vector>
 #include "tgp_common.cuh"
@@ -71,8 +72,9 @@ extern "C" int64_t tgp_batch_work_doubles(const int64_t* off, int32_t B) {
   return total;
 }
 
-// The per-call device tables: problem descriptors, kernel descriptors, the problem lists of every profile class and
-// (for the factorisation) one flag word per problem, in one stream-ordered allocation freed on the same stream.
+// The per-call device tables: problem descriptors, kernel descriptors, the problem lists of every profile class,
+// (for the factorisation) one flag word per problem and the caller's `extra` bytes, in one stream-ordered allocation
+// freed on the same stream.
 struct BatchTables {
   void* dev = nullptr;
   cudaStream_t st = nullptr;
@@ -80,6 +82,7 @@ struct BatchTables {
   KSumDesc* kd = nullptr;
   int32_t* list = nullptr;
   unsigned* flags = nullptr;
+  unsigned char* extra = nullptr;
   int32_t start[TGP_BATCH_NCLASS + 1] = {};   // class c owns list[start[c] .. start[c + 1])
   int64_t max_n[TGP_BATCH_NCLASS] = {}, max_m[TGP_BATCH_NCLASS] = {};
   ~BatchTables() {
@@ -90,14 +93,17 @@ struct BatchTables {
 static size_t align16(size_t n) { return (n + 15) & ~(size_t)15; }
 
 static int stage_tables(BatchTables& T, const std::vector<TgpBatchProb>& prob, const tgp_kernel_sum* ks,
-                        const std::vector<int>& cls, cudaStream_t st) {
+                        const std::vector<int>& cls, cudaStream_t st,
+                        const std::vector<unsigned char>& extra = std::vector<unsigned char>()) {
   const size_t B = prob.size();
   const size_t o_kd = align16(B * sizeof(TgpBatchProb));
   const size_t o_list = o_kd + align16(B * sizeof(KSumDesc));
   const size_t o_flags = o_list + align16(B * sizeof(int32_t));
-  const size_t bytes = o_flags + align16(B * sizeof(unsigned));
+  const size_t o_extra = o_flags + align16(B * sizeof(unsigned));
+  const size_t bytes = o_extra + align16(extra.size());
   std::vector<unsigned char> h(bytes, 0);
   memcpy(h.data(), prob.data(), B * sizeof(TgpBatchProb));
+  if (!extra.empty()) memcpy(h.data() + o_extra, extra.data(), extra.size());
   KSumDesc* kd = reinterpret_cast<KSumDesc*>(h.data() + o_kd);
   int32_t* list = reinterpret_cast<int32_t*>(h.data() + o_list);
   for (size_t b = 0; b < B; ++b) kd[b] = make_ksumdesc(&ks[b]);
@@ -120,6 +126,7 @@ static int stage_tables(BatchTables& T, const std::vector<TgpBatchProb>& prob, c
   T.kd = reinterpret_cast<KSumDesc*>(d + o_kd);
   T.list = reinterpret_cast<int32_t*>(d + o_list);
   T.flags = reinterpret_cast<unsigned*>(d + o_flags);
+  T.extra = d + o_extra;
   return TGP_OK;
 }
 
@@ -195,17 +202,15 @@ backward_batch_kernel(const TgpBatchProb* __restrict__ pr) {
   for (int64_t i = tid; i < N; i += BS_THREADS) p.alpha[i] = x[i];
 }
 
-extern "C" int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
-                                 const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
-                                 int32_t* info, void* stream) {
-  const char* fn = __func__;
-  int rc = check_batch(fn, off, B, ks);
-  if (rc) return rc;
-  BATCH_CHECK(X && y && yerr2 && work && alpha && out && info, "null pointer (X, y, yerr2, work, alpha, out, info)");
-  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
-  cudaStream_t st = (cudaStream_t)stream;
+// The chain of tgp_loglike_batch on checked arguments, with the tables staged into T (plus `extra` bytes) and their
+// host copy in prob.  out: 3 B doubles, or nullptr for T.extra's first 3 B doubles.
+static int loglike_batch_run(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                             const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
+                             int32_t* info, cudaStream_t st, BatchTables& T, std::vector<TgpBatchProb>& prob,
+                             const std::vector<unsigned char>& extra) {
+  int rc;
   const int ndim = ks[0].ndim;
-  std::vector<TgpBatchProb> prob(B);
+  prob.assign(B, TgpBatchProb{});
   std::vector<int> cls(B);
   std::vector<int64_t> Nh(B);
   int64_t woff = 0;
@@ -224,9 +229,9 @@ extern "C" int tgp_loglike_batch(const double* X, const double* y, const double*
     // the K build of tgp_kmat_sym_sum: the single-term kernel for one term without a white level
     cls[b] = (ks[b].nterms == 1 && ks[b].white == 0.0) ? ks[b].term[0].family : TGP_BATCH_SUM;
   }
-  BatchTables T;
-  rc = stage_tables(T, prob, ks, cls, st);
+  rc = stage_tables(T, prob, ks, cls, st, extra);
   if (rc) return rc;
+  if (!out) out = reinterpret_cast<double*>(T.extra);
   for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
     if (T.start[c + 1] == T.start[c]) continue;
     rc = tgp_batch_kmat_sym(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, T.max_n[c], st);
@@ -246,6 +251,77 @@ extern "C" int tgp_loglike_batch(const double* X, const double* y, const double*
     TGP_LAUNCH_CHECK();
   }
   return tgp_batch_loglike_finish(T.pr, B, want_alpha, info, out, st);
+}
+
+extern "C" int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                                 const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
+                                 int32_t* info, void* stream) {
+  const char* fn = __func__;
+  int rc = check_batch(fn, off, B, ks);
+  if (rc) return rc;
+  BATCH_CHECK(X && y && yerr2 && work && alpha && out && info, "null pointer (X, y, yerr2, work, alpha, out, info)");
+  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
+  BatchTables T;
+  std::vector<TgpBatchProb> prob;
+  return loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, want_alpha, out, info, (cudaStream_t)stream, T, prob,
+                           std::vector<unsigned char>());
+}
+
+extern "C" int64_t tgp_loglike_grad_sum_work_doubles(int64_t N, int32_t nterms);
+
+// Every problem's scratch block is even in length (the selected-inverse part, 2 TGP_OB^2 + TGP_OB even(N), exceeds
+// the (4 TGP_MAX_TERMS + 1) partials of N <= TGP_BATCH_MAX_N), so all blocks stay 16-byte aligned.
+extern "C" int64_t tgp_loglike_grad_batch_work_doubles(const int64_t* off, int32_t B) {
+  const char* fn = __func__;
+  if (B < 1) {
+    tgp_set_error("%s: invalid argument: B must be >= 1", fn);
+    return TGP_ERR_INVALID;
+  }
+  if (check_offsets(fn, "off", off, B, 1, TGP_BATCH_MAX_N)) return TGP_ERR_INVALID;
+  int64_t total = 0;
+  for (int32_t b = 0; b < B; ++b) total += tgp_loglike_grad_sum_work_doubles(off[b + 1] - off[b], TGP_MAX_TERMS);
+  return total;
+}
+
+extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off,
+                                      int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, double* out,
+                                      int32_t* info, double* scratch, void* stream) {
+  const char* fn = __func__;
+  int rc = check_batch(fn, off, B, ks);
+  if (rc) return rc;
+  BATCH_CHECK(X && y && yerr2 && work && alpha && out && info && scratch,
+              "null pointer (X, y, yerr2, work, alpha, out, info, scratch)");
+  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
+  BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  // extra tables: {logL, chi2, logdet} per problem, then the scratch block of every problem
+  const size_t o_scr = align16((size_t)B * 3 * sizeof(double));
+  std::vector<unsigned char> extra(o_scr + (size_t)B * sizeof(double*), 0);
+  double** scr_h = reinterpret_cast<double**>(extra.data() + o_scr);
+  int64_t soff = 0;
+  for (int32_t b = 0; b < B; ++b) {
+    scr_h[b] = scratch + soff;
+    soff += tgp_loglike_grad_sum_work_doubles(off[b + 1] - off[b], TGP_MAX_TERMS);
+  }
+  BatchTables T;
+  std::vector<TgpBatchProb> prob;
+  rc = loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, 1, nullptr, info, st, T, prob, extra);
+  if (rc) return rc;
+  const double* ll = reinterpret_cast<const double*>(T.extra);
+  double* const* scr = reinterpret_cast<double* const*>(T.extra + o_scr);
+  rc = tgp_batch_selinv(T.pr, scr, prob.data(), scr_h, B, st);
+  if (rc) return rc;
+  for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
+    if (T.start[c + 1] == T.start[c]) continue;
+    int max_terms = 1;   // a sum's CTAs of terms beyond its own exit
+    if (c == TGP_BATCH_SUM) {
+      for (int32_t b = 0; b < B; ++b) max_terms = ks[b].nterms > max_terms ? ks[b].nterms : max_terms;
+    }
+    rc = tgp_batch_grad_contract(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, scr, T.max_n[c],
+                                 max_terms, st);
+    if (rc) return rc;
+  }
+  return tgp_batch_grad_finish(T.pr, T.kd, scr, B, info, ll, out, st);
 }
 
 extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, const double* X, const int64_t* off,

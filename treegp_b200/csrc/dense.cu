@@ -354,88 +354,7 @@ template <bool FULL>
 __global__ void __launch_bounds__(TRSM_ROWS)
 trsm_panel_kernel(const double* __restrict__ L, int nb, int64_t ldl, double* __restrict__ B, int64_t M,
                   int64_t ldb) {
-  extern __shared__ __align__(16) double tsm[];
-  double* LsT = tsm;                 // NB x NB, LsT[j*NB + i] = L[i][j] (column j contiguous), zero padded
-  double* dinv = tsm + NB * NB;      // 1 / L[j][j]
-  double* Bs = dinv + NB;            // TRSM_ROWS x NB_PITCH (edge path only)
-  const int tid = threadIdx.x;
-  const int64_t r0 = (int64_t)blockIdx.x * TRSM_ROWS;
-  const int64_t gr = r0 + tid;
-  double x[NB];
-  if (FULL) {
-    if (gr < M) {
-      const double2* row = reinterpret_cast<const double2*>(B + gr * ldb);
-#pragma unroll
-      for (int j = 0; j < NB / 2; ++j) { const double2 v = row[j]; x[2 * j] = v.x; x[2 * j + 1] = v.y; }
-    } else {
-#pragma unroll
-      for (int j = 0; j < NB; ++j) x[j] = 0.0;
-    }
-  }
-  if (FULL && ((ldl & 1) == 0) && (((uintptr_t)L & 15) == 0)) {
-    // one batch of 32 independent 16-byte loads per thread: element pairs (i, 2c), (i, 2c+1) of the L tile
-    double2 lv[NB * NB / 2 / TRSM_ROWS];
-#pragma unroll
-    for (int q = 0; q < NB * NB / 2 / TRSM_ROWS; ++q) {
-      const int idx = tid + q * TRSM_ROWS;       // pair index: row i = idx / 32, column pair c = idx % 32
-      lv[q] = *reinterpret_cast<const double2*>(L + (int64_t)(idx >> 5) * ldl + 2 * (idx & 31));
-    }
-#pragma unroll
-    for (int q = 0; q < NB * NB / 2 / TRSM_ROWS; ++q) {
-      const int idx = tid + q * TRSM_ROWS;
-      const int i = idx >> 5, j = 2 * (idx & 31);
-      LsT[j * NB + i] = (j < i) ? lv[q].x : 0.0;
-      LsT[(j + 1) * NB + i] = (j + 1 < i) ? lv[q].y : 0.0;
-    }
-  } else {
-#pragma unroll 16
-    for (int idx = tid; idx < NB * NB; idx += TRSM_ROWS) {
-      const int i = idx / NB, j = idx % NB;  // coalesced along j
-      double v = 0.0;
-      if (i < nb && j < i) v = L[(int64_t)i * ldl + j];
-      LsT[j * NB + i] = v;
-    }
-  }
-  if (tid < NB) dinv[tid] = (tid < nb) ? 1.0 / L[(int64_t)tid * ldl + tid] : 1.0;
-  if (!FULL) {
-    for (int idx = tid; idx < TRSM_ROWS * NB; idx += TRSM_ROWS) {
-      const int r = idx / NB, j = idx % NB;
-      const int64_t g2 = r0 + r;
-      Bs[r * NB_PITCH + j] = (g2 < M && j < nb) ? B[g2 * ldb + j] : 0.0;
-    }
-  }
-  __syncthreads();
-  if (!FULL) {
-#pragma unroll
-    for (int j = 0; j < NB; ++j) x[j] = Bs[tid * NB_PITCH + j];
-  }
-#pragma unroll
-  for (int j = 0; j < NB; ++j) {
-    x[j] *= dinv[j];
-    const double nx = -x[j];
-#pragma unroll
-    for (int ip = ((j + 1) & ~1); ip < NB; ip += 2) {  // pairs (ip, ip+1); entries with i <= j are zero/skipped
-      const double2 l = *reinterpret_cast<const double2*>(LsT + j * NB + ip);
-      if (ip > j) x[ip] = fma(nx, l.x, x[ip]);
-      x[ip + 1] = fma(nx, l.y, x[ip + 1]);
-    }
-  }
-  if (FULL) {
-    if (gr < M) {
-      double2* row = reinterpret_cast<double2*>(B + gr * ldb);
-#pragma unroll
-      for (int j = 0; j < NB / 2; ++j) row[j] = make_double2(x[2 * j], x[2 * j + 1]);
-    }
-  } else {
-#pragma unroll
-    for (int j = 0; j < NB; ++j) Bs[tid * NB_PITCH + j] = x[j];
-    __syncthreads();
-    for (int idx = tid; idx < TRSM_ROWS * NB; idx += TRSM_ROWS) {
-      const int r = idx / NB, j = idx % NB;
-      const int64_t g2 = r0 + r;
-      if (g2 < M && j < nb) B[g2 * ldb + j] = Bs[r * NB_PITCH + j];
-    }
-  }
+#include "trsm_panel_body.cuh"
 }
 
 static int trsm_panel_launch(const double* L, int nb, int64_t ldl, double* B, int64_t M, int64_t ldb,
@@ -1456,6 +1375,104 @@ loglike_batch_finish_kernel(const TgpBatchProb* __restrict__ pr, int want_alpha,
 int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int want_alpha, const int32_t* info, double* out,
                              cudaStream_t st) {
   loglike_batch_finish_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, want_alpha, info, out);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// ============================================================================================
+// Selected inverse of a batch (tgp_batch_selinv in selinv.cu): the halving leaves and the DMMA products of step s of
+// selinv_run, on a grid of (problem, CTA of the single launch); CTAs of problems without that launch exit.  Scratch
+// of a problem as selinv_run lays it out: -W^T, W^T (TGP_OB x TGP_OB each), T^T (TGP_OB x even(N)).
+// ============================================================================================
+// grid: (CTA of the single launch, leaf blockIdx.y of the launch's table).  The operands come from the parameter bank,
+// as the single kernel's do: that keeps them out of the registers, which the row solve of the FULL path fills.
+template <bool FULL>
+__global__ void __launch_bounds__(TRSM_ROWS)
+selinv_leaf_batch_kernel(const __grid_constant__ TgpLeafLaunch p) {
+  const TgpLeafArgs& a = p.a[blockIdx.y];
+  if ((int64_t)blockIdx.x * TRSM_ROWS >= a.M) return;
+  const double* const L = a.L;
+  double* const B = a.B;
+  const int64_t ldl = a.ldl, M = a.M, ldb = a.ldb;
+  const int nb = a.nb;
+#include "trsm_panel_body.cuh"
+}
+
+int tgp_batch_selinv_leaves(const TgpLeafArgs* leaves, int32_t n, bool full, cudaStream_t st) {
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once)) {
+    TGP_CUDA(cudaFuncSetAttribute(selinv_leaf_batch_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  TRSM_SMEM));
+    TGP_CUDA(cudaFuncSetAttribute(selinv_leaf_batch_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  TRSM_SMEM));
+  }
+  for (int32_t i0 = 0; i0 < n; i0 += TGP_LEAF_GROUP) {
+    TgpLeafLaunch p;
+    const int32_t cnt = std::min(n - i0, TGP_LEAF_GROUP);
+    int64_t mmax = 0;
+    for (int32_t i = 0; i < cnt; ++i) {
+      p.a[i] = leaves[i0 + i];
+      mmax = std::max(mmax, p.a[i].M);
+    }
+    const dim3 grid((unsigned)tgp_cdiv(mmax, TRSM_ROWS), (unsigned)cnt);
+    if (full) selinv_leaf_batch_kernel<true><<<grid, TRSM_ROWS, TRSM_SMEM, st>>>(p);
+    else selinv_leaf_batch_kernel<false><<<grid, TRSM_ROWS, TRSM_SMEM, st>>>(p);
+    TGP_LAUNCH_CHECK();
+  }
+  return TGP_OK;
+}
+
+// grid: (problem, row tile * tiles_n + column tile) of the product `op` (batch.cuh) of step s
+__global__ void __launch_bounds__(GEMM_THREADS, 2)
+selinv_gemm_batch_kernel(const TgpBatchProb* __restrict__ pr, double* const* __restrict__ scr, int s, int op,
+                         int leaf, int tiles_n) {
+  const int b = blockIdx.x;
+  TgpSelStep g;
+  if (!tgp_selinv_step(pr[b].N, s, g)) return;
+  int64_t M, Nc, Kd;
+  if (!tgp_selinv_gemm_shape(g, op, leaf, M, Nc, Kd)) return;
+  const int64_t m0 = (int64_t)(blockIdx.y / tiles_n) * BM, n0 = (int64_t)(blockIdx.y % tiles_n) * 64;
+  if (m0 >= M || n0 >= Nc) return;
+  const int64_t ld = pr[b].ld, ldt = (pr[b].N + 1) & ~(int64_t)1;
+  double* A = pr[b].A;
+  double* NWT = scr[b];
+  double* WT = NWT + TGP_OB * TGP_OB;
+  double* TT = NWT + 2 * TGP_OB * TGP_OB;
+  double* Akk = A + g.k * ld + g.k;
+  double* L21 = A + g.c1 * ld + g.k;
+  double* C;
+  const double *X, *Y;
+  int64_t ldc = ld, ldx = TGP_OB, ldy = ld;
+  int lower = 0;
+  switch (op) {
+    case TGP_SEL_TT: C = TT; ldc = ldt; X = NWT; Y = L21; break;                                       // T^T = W^T L21^T
+    case TGP_SEL_ZRJ: C = L21; X = A + g.c1 * ld + g.c1; ldx = ld; Y = TT; ldy = ldt; break;           // -Z[R, R] T
+    case TGP_SEL_WTW: C = Akk; X = NWT; Y = WT; ldy = TGP_OB; lower = 1; break;                          // + W^T W
+    case TGP_SEL_TZ: C = Akk; X = TT; ldx = ldt; Y = A + g.k * ld + g.c1; lower = 1; break;           // - T^T Z[J, R]
+    default: {   // B2 -= B1 L21^T of trsm_rows_halving on the node [o, o + n) split at h
+      int64_t o, h, n;
+      tgp_halving_node(g.w, leaf, o, h, n);
+      C = NWT + o + h;
+      ldc = TGP_OB;
+      X = NWT + o;
+      Y = Akk + (o + h) * ld + o;
+    }
+  }
+  gemm_nt_sub_tile<64, 4, 2>(C, M, Nc, ldc, X, ldx, Y, ldy, Kd, lower, m0, n0);
+}
+
+int tgp_batch_selinv_gemm(const TgpBatchProb* pr, double* const* scr, int32_t B, int s, int op, int leaf,
+                          int tiles_n, int64_t tiles, cudaStream_t st) {
+  constexpr int GSMEM = STAGES * (BM + 64) * BK * 8;
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once)) {
+    TGP_CUDA(cudaFuncSetAttribute(selinv_gemm_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM));
+    TGP_CUDA(cudaFuncSetAttribute(selinv_gemm_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+  }
+  TGP_CHECK_ARG(tiles <= 65535, "too many tiles for one launch");
+  selinv_gemm_batch_kernel<<<dim3((unsigned)B, (unsigned)tiles), GEMM_THREADS, GSMEM, st>>>(pr, scr, s, op, leaf,
+                                                                                          tiles_n);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

@@ -16,9 +16,11 @@
 // over the lower triangle inside the envelope: with w_ij = alpha_i alpha_j - Z_ij and K_ij = a f(q_ij),
 //   d logL / d ln a = 1/2 sum_ij w_ij a f(q_ij),   d logL / d m_uv = 1/2 sum_ij w_ij a f'(q_ij) d q_ij / d m_uv.
 #include <string.h>
+#include <algorithm>
 #include "tgp_common.cuh"
 #include "profile_dq.cuh"
 #include "profile_policy.cuh"
+#include "batch.cuh"
 
 extern "C" int tgp_trsm_rows(const double* L, int64_t N, int64_t ld, double* B, int64_t M, int64_t ldb, void* stream);
 extern "C" int tgp_gemm_nt_sub(double* C, int64_t M, int64_t Nc, int64_t ldc, const double* A, int64_t lda,
@@ -87,11 +89,11 @@ __global__ void negate_kernel(const double* __restrict__ S, double* __restrict__
 
 // dst[c][r] = src[r][c] for the rows x cols block src (both with pitch ld).  lower_only: src == dst is a square
 // diagonal block whose strict lower triangle is mirrored into its upper triangle (disjoint entries: no race).
-__global__ void __launch_bounds__(256)
-mirror_kernel(const double* __restrict__ src, double* __restrict__ dst, int64_t rows, int64_t cols, int64_t ld,
-              int lower_only) {
+// The 32 x 32 tile whose top-left corner is (r0, c0).
+__device__ __forceinline__ void mirror_body(const double* __restrict__ src, double* __restrict__ dst, int64_t rows,
+                                            int64_t cols, int64_t ld, int lower_only, const int64_t r0,
+                                            const int64_t c0) {
   __shared__ double t[32][33];
-  const int64_t r0 = (int64_t)blockIdx.y * 32, c0 = (int64_t)blockIdx.x * 32;
   if (lower_only && c0 > r0) return;
   const int tx = threadIdx.x, ty = threadIdx.y;   // 32 x 8
 #pragma unroll
@@ -105,6 +107,12 @@ mirror_kernel(const double* __restrict__ src, double* __restrict__ dst, int64_t 
     const int64_t c = c0 + ty + 8 * i, r = r0 + tx;   // write row c of dst, coalesced along r
     if (r < rows && c < cols && (!lower_only || c < r)) dst[c * ld + r] = t[tx][ty + 8 * i];
   }
+}
+
+__global__ void __launch_bounds__(256)
+mirror_kernel(const double* __restrict__ src, double* __restrict__ dst, int64_t rows, int64_t cols, int64_t ld,
+              int lower_only) {
+  mirror_body(src, dst, rows, cols, ld, lower_only, (int64_t)blockIdx.y * 32, (int64_t)blockIdx.x * 32);
 }
 
 static int mirror_launch(const double* src, double* dst, int64_t rows, int64_t cols, int64_t ld, int lower_only,
@@ -195,125 +203,14 @@ __global__ void __launch_bounds__(GT_THREADS)
 grad_contract_kernel(const double* __restrict__ X, int64_t N, P prof, const double* __restrict__ Z, int64_t ld,
                      const double* __restrict__ alpha, const int64_t* __restrict__ re_dev,
                      double* __restrict__ partials, const double* __restrict__ phi_g) {
-  constexpr int RM = OutputsOf<P>::kR;
-  __shared__ double xr[GT], yr[GT], ar[GT * RM], xc[GT], yc[GT], ac[GT * RM];
-  __shared__ double red[GT_THREADS / 32][P::kSum ? 5 : 4];
-  __shared__ double phi_s[P::kPhiSize];
-  const KDesc& kd = prof.grad_term();
-  const int64_t t = blockIdx.x;
-  int64_t I = (int64_t)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
-  while (I * (I + 1) / 2 > t) --I;
-  while ((I + 1) * (I + 2) / 2 <= t) ++I;
-  const int64_t J = t - I * (I + 1) / 2;
-  const int64_t r0 = I * GT, c0 = J * GT;
-  const int64_t rend = re_dev ? re_dev[c0 / TGP_OB] : N;   // one past the last envelope row of this block column
-  const int tid = threadIdx.x;
-  if (r0 >= rend) {
-    if (tid < 4) partials[prof.partial(t, tid)] = 0.0;
-    if constexpr (P::kSum) {
-      if (tid == 4 && blockIdx.y == 0) partials[prof.white_partial(t)] = 0.0;
-    }
-    return;
-  }
-  if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
-  if (tid < GT) {
-    const int64_t r = r0 + tid;
-    const bool ok = r < N;
-    xr[tid] = ok ? X[r * kd.ndim] : 0.0;
-    yr[tid] = (ok && kd.ndim == 2) ? X[r * 2 + 1] : 0.0;
-    if constexpr (RM > 1) {
-      for (int c = 0; c < prof.nrhs; ++c) ar[tid * RM + c] = ok ? alpha[r * prof.nrhs + c] : 0.0;
-    } else {
-      ar[tid] = ok ? alpha[r] : 0.0;
-    }
-  } else if (tid < 2 * GT) {
-    const int l = tid - GT;
-    const int64_t c = c0 + l;
-    const bool ok = c < N;
-    xc[l] = ok ? X[c * kd.ndim] : 0.0;
-    yc[l] = (ok && kd.ndim == 2) ? X[c * 2 + 1] : 0.0;
-    if constexpr (RM > 1) {
-      for (int j = 0; j < prof.nrhs; ++j) ac[l * RM + j] = ok ? alpha[c * prof.nrhs + j] : 0.0;
-    } else {
-      ac[l] = ok ? alpha[c] : 0.0;
-    }
-  }
-  __syncthreads();
-  const int lane = tid & 31, warp = tid >> 5;
-  double s[4] = {0.0, 0.0, 0.0, 0.0};
-  double sw = 0.0;   // sums: the white column
-#pragma unroll(P::kHeavy ? 1 : GT / 8)
-  for (int rr = 0; rr < GT / 8; ++rr) {
-    const int rl = warp + 8 * rr;
-    const int64_t rg = r0 + rl;
-    if (rg >= N || rg >= rend) continue;
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const int cl = 2 * lane + h;
-      const int64_t cg = c0 + cl;
-      if (cg > rg) continue;
-      const double dx = xr[rl] - xc[cl], dy = yr[rl] - yc[cl];
-      const double q = tgp_qform(kd, dx, dy);
-      double wij;
-      if constexpr (RM > 1) {
-        const double* a = ar + rl * RM;
-        const double* b = ac + cl * RM;
-        double aa = a[0] * b[0];
-        for (int c = 1; c < prof.nrhs; ++c) aa = fma(a[c], b[c], aa);
-        wij = (rg == cg ? 1.0 : 2.0) * (aa - (double)prof.nrhs * Z[rg * ld + cg]);
-      } else {
-        wij = (rg == cg ? 1.0 : 2.0) * (ar[rl] * ac[cl] - Z[rg * ld + cg]);
-      }
-      double f = prof.f(kd, q, phi_s);
-      // K(X, X) of the von Karman kernels is 0 between distinct coincident points (kmat.cu, kernels.py:253-262)
-      if (prof.vk(kd) && q == 0.0 && rg != cg) f = 0.0;
-      if constexpr (P::kSum) {
-        if (rg == cg) sw += wij;
-      }
-      s[0] = fma(wij, kd.amp * f, s[0]);
-      if (q > 0.0) {
-        const double d = wij * kd.amp * prof.fdq(kd, q, phi_s);
-        s[1] = fma(d, dx * dx, s[1]);
-        s[2] = fma(d, 2.0 * dx * dy, s[2]);
-        s[3] = fma(d, dy * dy, s[3]);
-      }
-    }
-  }
-#pragma unroll
-  for (int c = 0; c < 4; ++c) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) s[c] += __shfl_xor_sync(0xffffffffu, s[c], o);
-  }
-  if constexpr (P::kSum) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) sw += __shfl_xor_sync(0xffffffffu, sw, o);
-    if (lane == 0) red[warp][4] = sw;
-  }
-  if (lane == 0) {
-#pragma unroll
-    for (int c = 0; c < 4; ++c) red[warp][c] = s[c];
-  }
-  __syncthreads();
-  if (tid < 4) {
-    double v = 0.0;
-    for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi][tid];
-    partials[prof.partial(t, tid)] = v;
-  }
-  if constexpr (P::kSum) {
-    if (tid == 4 && blockIdx.y == 0) {
-      double v = 0.0;
-      for (int wi = 0; wi < GT_THREADS / 32; ++wi) v += red[wi][4];
-      partials[prof.white_partial(t)] = prof.desc.white * v;
-    }
-  }
+#include "grad_contract_body.cuh"
 }
 
 // out[3 .. 3 + NC - 1] = 1/2 the tile sums of the NC partial columns in tile order; 0 when the factorisation failed
 // (out[0] is then -inf already).  NC = 4 for one term, 4 nterms + 1 for a sum.
 template <int NC>
-__global__ void __launch_bounds__(1024)
-grad_finish_kernel(const double* __restrict__ partials, int64_t ntiles, const int32_t* __restrict__ info,
-                   double* __restrict__ out) {
+__device__ __forceinline__ void grad_finish_body(const double* __restrict__ partials, int64_t ntiles,
+                                                 const int32_t* __restrict__ info, double* __restrict__ out) {
   __shared__ double red[32][NC];
   double s[NC];
 #pragma unroll
@@ -338,6 +235,13 @@ grad_finish_kernel(const double* __restrict__ partials, int64_t ntiles, const in
     for (int wi = 0; wi < 32; ++wi) v += red[wi][threadIdx.x];
     out[3 + threadIdx.x] = (*info != 0) ? 0.0 : 0.5 * v;
   }
+}
+
+template <int NC>
+__global__ void __launch_bounds__(1024)
+grad_finish_kernel(const double* __restrict__ partials, int64_t ntiles, const int32_t* __restrict__ info,
+                   double* __restrict__ out) {
+  grad_finish_body<NC>(partials, ntiles, info, out);
 }
 
 static int grad_args(const double* X, const double* y, int64_t N, double* work, int64_t ld, const double* alpha,
@@ -442,4 +346,211 @@ extern "C" int tgp_loglike_grad_multi(const double* X, const double* Y, int32_t 
   }
   return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
                    row_end, scratch, st, r);
+}
+
+// ---- batches of independent problems (tgp_loglike_grad_batch) ---------------------------------------------------
+// The selected inverse, contraction and finish above on every problem of a batch: each launch of selinv_run's
+// schedule runs its body on a grid of (problem, CTA), step s handling block column nb_b - 1 - s of problem b
+// (batch.cuh), so that every problem starts at step 0; CTAs of problems without that launch exit.  The fills and
+// mirrors only move values, and the products and the halving solve are the single call's tile bodies (dense.cu), so Z
+// is tgp_selinv's bit for bit.
+
+// 0: -W^T = -I, 1: W^T = -(-W^T), 2: T^T = 0, 3: Z[R, J] = 0, 4: Z[J, J] = 0 (the memsets of selinv_run)
+enum { SEL_NEG_I = 0, SEL_NEGATE = 1, SEL_ZERO_TT = 2, SEL_ZERO_ZRJ = 3, SEL_ZERO_ZJJ = 4 };
+__global__ void __launch_bounds__(256)
+selinv_fill_batch_kernel(const TgpBatchProb* __restrict__ pr, double* const* __restrict__ scr, int s, int op) {
+  const int b = blockIdx.x;
+  TgpSelStep g;
+  if (!tgp_selinv_step(pr[b].N, s, g)) return;
+  const int64_t ld = pr[b].ld, ldt = (pr[b].N + 1) & ~(int64_t)1;
+  double* NWT = scr[b];
+  double* dst = NWT;
+  int64_t rows = g.w, cols = g.w, pitch = TGP_OB;
+  switch (op) {
+    case SEL_NEGATE: dst = NWT + TGP_OB * TGP_OB; break;
+    case SEL_ZERO_TT: dst = NWT + 2 * TGP_OB * TGP_OB; cols = g.m; pitch = ldt; break;
+    case SEL_ZERO_ZRJ: dst = pr[b].A + g.c1 * ld + g.k; rows = g.m; pitch = ld; break;
+    case SEL_ZERO_ZJJ: dst = pr[b].A + g.k * ld + g.k; pitch = ld; break;
+    default: break;
+  }
+  for (int64_t idx = blockIdx.y * (int64_t)blockDim.x + threadIdx.x; idx < rows * cols;
+       idx += (int64_t)gridDim.y * blockDim.x) {
+    const int64_t r = idx / cols, c = idx % cols;
+    double v = 0.0;
+    if (op == SEL_NEG_I) v = (r == c) ? -1.0 : 0.0;
+    else if (op == SEL_NEGATE) v = -NWT[r * TGP_OB + c];
+    dst[r * pitch + c] = v;
+  }
+}
+
+// 0: Z[J, R] = Z[R, J]^T, 1: the upper triangle of Z[J, J].  grid: (problem, row tile * tiles_c + column tile)
+__global__ void __launch_bounds__(256)
+selinv_mirror_batch_kernel(const TgpBatchProb* __restrict__ pr, int s, int op, int tiles_c) {
+  const int b = blockIdx.x;
+  TgpSelStep g;
+  if (!tgp_selinv_step(pr[b].N, s, g)) return;
+  const int64_t ld = pr[b].ld, rows = op == 0 ? g.m : g.w;
+  const int64_t r0 = (int64_t)(blockIdx.y / tiles_c) * 32, c0 = (int64_t)(blockIdx.y % tiles_c) * 32;
+  if (r0 >= rows || c0 >= g.w) return;
+  double* A = pr[b].A;
+  if (op == 0) mirror_body(A + g.c1 * ld + g.k, A + g.k * ld + g.c1, rows, g.w, ld, 0, r0, c0);
+  else mirror_body(A + g.k * ld + g.k, A + g.k * ld + g.k, rows, g.w, ld, 1, r0, c0);
+}
+
+int tgp_batch_selinv(const TgpBatchProb* pr, double* const* scr, const TgpBatchProb* prob_h, double* const* scr_h,
+                     int32_t B, cudaStream_t st) {
+  std::vector<int64_t> Nh(B);
+  int smax = 0;
+  for (int32_t b = 0; b < B; ++b) {
+    Nh[b] = prob_h[b].N;
+    smax = std::max(smax, (int)tgp_cdiv(Nh[b], TGP_OB));
+  }
+  std::vector<TgpLeafArgs> full, edge;
+  auto fill = [&](int s, int op, int64_t elems) -> int {
+    if (elems <= 0) return TGP_OK;
+    const unsigned ctas = (unsigned)std::min<int64_t>(tgp_cdiv(elems, 256), 64);
+    selinv_fill_batch_kernel<<<dim3((unsigned)B, ctas), 256, 0, st>>>(pr, scr, s, op);
+    TGP_LAUNCH_CHECK();
+    return TGP_OK;
+  };
+  // the largest launch of product `op` over the problems of step s
+  auto gemm = [&](int s, int op, int leaf) -> int {
+    int64_t tm = 0, tn = 0;
+    for (int32_t b = 0; b < B; ++b) {
+      TgpSelStep g;
+      int64_t M, Nc, Kd;
+      if (!tgp_selinv_step(Nh[b], s, g) || !tgp_selinv_gemm_shape(g, op, leaf, M, Nc, Kd)) continue;
+      tm = std::max(tm, tgp_cdiv(M, 128));
+      tn = std::max(tn, tgp_cdiv(Nc, 64));
+    }
+    if (tm == 0) return TGP_OK;
+    return tgp_batch_selinv_gemm(pr, scr, B, s, op, leaf, (int)tn, tm * tn, st);
+  };
+  auto mirror = [&](int s, int op, int64_t rows, int64_t cols) -> int {
+    if (rows <= 0 || cols <= 0) return TGP_OK;
+    const int64_t tc = tgp_cdiv(cols, 32), tiles = tgp_cdiv(rows, 32) * tc;
+    TGP_CHECK_ARG(tiles <= 65535, "too many tiles for one launch");
+    selinv_mirror_batch_kernel<<<dim3((unsigned)B, (unsigned)tiles), dim3(32, 8), 0, st>>>(pr, s, op, (int)tc);
+    TGP_LAUNCH_CHECK();
+    return TGP_OK;
+  };
+  int rc;
+  for (int s = 0; s < smax; ++s) {
+    int64_t wmax = 0, mmax = 0;
+    for (int32_t b = 0; b < B; ++b) {
+      TgpSelStep g;
+      if (!tgp_selinv_step(Nh[b], s, g)) continue;
+      wmax = std::max(wmax, g.w);
+      mmax = std::max(mmax, g.m);
+    }
+    if ((rc = fill(s, SEL_NEG_I, wmax * wmax))) return rc;
+    // -W^T: rows of -I times L11^-T by halving, leaf, gemm, leaf, ..., leaf for every problem
+    const int nleaves = (int)tgp_cdiv(wmax, 64);
+    for (int i = 0; i < nleaves; ++i) {
+      full.clear();
+      edge.clear();
+      for (int32_t b = 0; b < B; ++b) {   // leaf i of problem b, on the path trsm_panel_launch takes for it
+        TgpSelStep g;
+        const int64_t c0 = 64 * (int64_t)i;
+        if (!tgp_selinv_step(Nh[b], s, g) || g.w <= c0) continue;
+        const int64_t ld = prob_h[b].ld;
+        const int nb = (int)std::min<int64_t>(g.w - c0, 64);
+        (nb == 64 ? full : edge).push_back(
+            TgpLeafArgs{prob_h[b].A + (g.k + c0) * ld + g.k + c0, scr_h[b] + c0, ld, g.w, TGP_OB, nb});
+      }
+      if ((rc = tgp_batch_selinv_leaves(full.data(), (int32_t)full.size(), true, st))) return rc;
+      if ((rc = tgp_batch_selinv_leaves(edge.data(), (int32_t)edge.size(), false, st))) return rc;
+      if (i + 1 < nleaves && (rc = gemm(s, TGP_SEL_HALVE, i))) return rc;
+    }
+    if ((rc = fill(s, SEL_NEGATE, wmax * wmax))) return rc;
+    if (mmax > 0) {
+      if ((rc = fill(s, SEL_ZERO_TT, wmax * mmax))) return rc;
+      if ((rc = gemm(s, TGP_SEL_TT, 0))) return rc;
+      if ((rc = fill(s, SEL_ZERO_ZRJ, wmax * mmax))) return rc;
+      if ((rc = gemm(s, TGP_SEL_ZRJ, 0))) return rc;
+      if ((rc = mirror(s, 0, mmax, wmax))) return rc;
+    }
+    if ((rc = fill(s, SEL_ZERO_ZJJ, wmax * wmax))) return rc;
+    if ((rc = gemm(s, TGP_SEL_WTW, 0))) return rc;
+    if (mmax > 0 && (rc = gemm(s, TGP_SEL_TZ, 0))) return rc;
+    if ((rc = mirror(s, 1, wmax, wmax))) return rc;
+  }
+  return TGP_OK;
+}
+
+// grid: (tile, term, problem of the list); the single call's contraction on each problem, Z in its workspace block and
+// the tile partials at the front of its scratch.  The problem's profile is staged in shared memory: the body indexes a
+// sum's terms by blockIdx.y, which a copy in registers could only do from the stack.
+template <class P>
+__global__ void __launch_bounds__(GT_THREADS)
+grad_contract_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* __restrict__ descs,
+                           const int32_t* __restrict__ list, double* const* __restrict__ scr,
+                           const double* __restrict__ phi_g) {
+  const int b = list[blockIdx.z];
+  const int64_t N = pr[b].N, nt = (N + GT - 1) / GT;
+  if ((int64_t)blockIdx.x >= nt * (nt + 1) / 2) return;
+  if (P::kSum && (int)blockIdx.y >= descs[b].nterms) return;
+  __shared__ P prof_s;   // P holds one descriptor: the sum's, or a family's single term
+  static_assert(sizeof(prof_s.desc) == sizeof(P) && sizeof(P) % 4 == 0, "a profile is its descriptor");
+  {
+    const int* src = reinterpret_cast<const int*>(P::kSum ? (const void*)&descs[b] : (const void*)&descs[b].term[0]);
+    int* dst = reinterpret_cast<int*>(&prof_s);
+    for (int i = threadIdx.x; i < (int)(sizeof(P) / 4); i += GT_THREADS) dst[i] = src[i];
+  }
+  __syncthreads();
+  const P& prof = prof_s;
+  const double* __restrict__ X = pr[b].X;
+  const double* __restrict__ Z = pr[b].A;
+  const double* __restrict__ alpha = pr[b].alpha;
+  const int64_t ld = pr[b].ld;
+  const int64_t* __restrict__ re_dev = nullptr;
+  double* __restrict__ partials = scr[b];
+#include "grad_contract_body.cuh"
+}
+
+int tgp_batch_grad_contract(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
+                            double* const* scr, int64_t max_n, int max_terms, cudaStream_t st) {
+  const int64_t ntiles = grad_tiles(max_n);
+  TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
+  const double* phi = tgp_phi_device();
+  for (int32_t z0 = 0; z0 < count; z0 += 65535) {   // gridDim.z <= 65535
+    const dim3 grid((unsigned)ntiles, (unsigned)max_terms, (unsigned)std::min(count - z0, 65535));
+    if (cls == TGP_BATCH_SUM) {
+      grad_contract_batch_kernel<SumProfile><<<grid, GT_THREADS, 0, st>>>(pr, kd, list + z0, scr, phi);
+    } else {
+      TGP_FAMILY_SWITCH(cls, (grad_contract_batch_kernel<FamilyProfile<FAM>><<<grid, GT_THREADS, 0, st>>>(
+                                 pr, kd, list + z0, scr, phi)));
+    }
+    TGP_LAUNCH_CHECK();
+  }
+  return TGP_OK;
+}
+
+// One CTA per problem: grad_finish_kernel with the single call's NC, then the rest of the problem's output slice.
+__global__ void __launch_bounds__(1024)
+grad_finish_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* __restrict__ kd,
+                         double* const* __restrict__ scr, const int32_t* __restrict__ info,
+                         const double* __restrict__ ll, double* __restrict__ out) {
+  const int b = blockIdx.x;
+  const int nterms = kd[b].nterms;
+  const int nc = (nterms == 1 && kd[b].white == 0.0) ? 4 : 4 * nterms + 1;   // one term: d / d ln white = 0
+  const int64_t nt = (pr[b].N + GT - 1) / GT, ntiles = nt * (nt + 1) / 2;
+  double* o = out + (int64_t)b * TGP_GRAD_BATCH_OUT;
+  const int tid = threadIdx.x;
+  if (tid < 3) o[tid] = ll[3 * (int64_t)b + tid];
+  else if (tid >= 3 + nc && tid < TGP_GRAD_BATCH_OUT) o[tid] = 0.0;
+  switch (nc) {
+    case 4: grad_finish_body<4>(scr[b], ntiles, info + b, o); break;
+    case 5: grad_finish_body<5>(scr[b], ntiles, info + b, o); break;
+    case 9: grad_finish_body<9>(scr[b], ntiles, info + b, o); break;
+    case 13: grad_finish_body<13>(scr[b], ntiles, info + b, o); break;
+    default: grad_finish_body<4 * TGP_MAX_TERMS + 1>(scr[b], ntiles, info + b, o); break;
+  }
+}
+
+int tgp_batch_grad_finish(const TgpBatchProb* pr, const KSumDesc* kd, double* const* scr, int32_t B,
+                          const int32_t* info, const double* ll, double* out, cudaStream_t st) {
+  grad_finish_batch_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, kd, scr, info, ll, out);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
 }

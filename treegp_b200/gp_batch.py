@@ -17,17 +17,19 @@ import torch
 from scipy import optimize
 
 from . import _cabi, backend
-from .kernels import descriptor_params, eval_kernel, lower
+from .kernels import descriptor_params, eval_kernel, lower, lower_jacobian
+from .log_likelihood import log_likelihood
 from .two_pcf import two_pcf
 
 OPTIMIZERS = ["anisotropic", "two-pcf", "log-likelihood", "none"]
 _ABORT = object()
 
 
-def lockstep_minimize(evaluate, x0s):
+def lockstep_minimize(evaluate, x0s, jac=False):
     """Run one ``scipy.optimize.minimize(f_b, x0s[b], method="L-BFGS-B")`` per problem, exactly as
     ``log_likelihood.optimizer`` does (no bounds, scipy's forward-difference gradient), with the objective values of
-    all problems computed together.
+    all problems computed together.  With jac=True each search is ``minimize(f_b, x0s[b], method="L-BFGS-B",
+    jac=True)`` and ``evaluate`` returns one (value, gradient) pair per request, as with ANALYTIC_GRADIENT.
 
     Each search runs in a worker thread whose objective only posts its theta and waits.  The calling thread collects
     one request from every live search, calls ``evaluate(indices, thetas)`` (a sequence of objective values, one per
@@ -48,7 +50,7 @@ def lockstep_minimize(evaluate, x0s):
             return v
 
         try:
-            requests.put(("done", b, optimize.minimize(fun, x0s[b], method="L-BFGS-B")["x"]))
+            requests.put(("done", b, optimize.minimize(fun, x0s[b], method="L-BFGS-B", jac=jac)["x"]))
         except BaseException as e:  # noqa: BLE001  (handed to the calling thread, which re-raises)
             requests.put(("error", b, e))
 
@@ -73,7 +75,7 @@ def lockstep_minimize(evaluate, x0s):
                 if len(values) != len(pending):
                     raise ValueError("evaluate returned %d values for %d requests" % (len(values), len(pending)))
                 for (b, _), v in zip(pending, values):
-                    replies[b].put(float(v))
+                    replies[b].put((float(v[0]), np.array(v[1], dtype=float)) if jac else float(v))
                 pending = []
     except BaseException as e:  # noqa: BLE001
         error = e
@@ -181,41 +183,68 @@ class GPInterpolationBatch(object):
             self._dev = (X, y, e2, sizes, backend.batch_offsets(sizes))
         return self._dev
 
-    def _loglike(self, indices, kernels):
-        """logL of the problems `indices` for `kernels`: one batched call (chunked by WORK_BUDGET) for those whose
-        descriptor is finite, -inf without a launch for the others (as log_likelihood.log_likelihood)."""
+    def _batched(self, indices, descs, call, name):
+        """One batched device call `call` (backend.loglike_batch or loglike_grad_batch, chunked by WORK_BUDGET) over
+        the problems `indices` whose descriptor in `descs` is finite; the others launch nothing (as
+        log_likelihood.log_likelihood).  Returns (the positions in `indices` that ran, their out rows on the host)."""
         X, y, e2, sizes, off = self._device_data()
-        ndim = X.shape[1]
-        values = np.full(len(indices), -np.inf)
-        run, descs = [], []
-        for i, (b, k) in enumerate(zip(indices, kernels)):
-            desc = lower(k, ndim)
-            if np.all(np.isfinite(descriptor_params(desc))):
-                run.append(i)
-                descs.append(desc)
+        run = [i for i, d in enumerate(descs) if np.all(np.isfinite(descriptor_params(d)))]
         if not run:
-            return values
+            return run, None
         probs = [indices[i] for i in run]
         if probs == list(range(len(sizes))):
             Xr, yr, er = X, y, e2
         else:
             rows = torch.as_tensor(np.concatenate([np.arange(off[b], off[b + 1]) for b in probs]), device=X.device)
             Xr, yr, er = X[rows].contiguous(), y[rows].contiguous(), e2[rows].contiguous()
-        out, info, _ = backend.loglike_batch(Xr, yr, er, [sizes[b] for b in probs], descs,
-                                             budget_bytes=self.WORK_BUDGET)
-        ll = out[:, 0].cpu().numpy()
-        if np.any(ll != ll):   # NaN marks info < 0: an internal synchronisation timeout, never a -inf
-            raise _cabi.TgpError("tgp_loglike_batch: internal synchronisation timed out (info = %r)"
-                                 % info.cpu().numpy().tolist())
-        values[run] = ll
+        out, info, _ = call(Xr, yr, er, [sizes[b] for b in probs], [descs[i] for i in run],
+                            budget_bytes=self.WORK_BUDGET)
+        out = out.cpu().numpy()
+        if np.any(out[:, 0] != out[:, 0]):   # NaN marks info < 0: an internal synchronisation timeout, never a -inf
+            raise _cabi.TgpError("%s: internal synchronisation timed out (info = %r)"
+                                 % (name, info.cpu().numpy().tolist()))
+        return run, out
+
+    def _loglike(self, indices, kernels):
+        """logL of the problems `indices` for `kernels`: one batched call for those whose descriptor is finite, -inf
+        without a launch for the others."""
+        ndim = self._device_data()[0].shape[1]
+        values = np.full(len(indices), -np.inf)
+        run, out = self._batched(indices, [lower(k, ndim) for k in kernels], backend.loglike_batch,
+                                 "tgp_loglike_batch")
+        if run:
+            values[run] = out[:, 0]
         return values
 
+    def _loglike_and_gradient(self, indices, kernels):
+        """(logL, d logL / d theta) of the problems `indices` for `kernels`: one batched value-and-gradient call
+        (tgp_loglike_grad_batch) for those whose descriptor is finite; -inf and a zero gradient without a launch for
+        the others, and -inf with a zero gradient where K is not positive definite (as
+        log_likelihood.log_likelihood_and_gradient).  A list of (value, gradient) pairs."""
+        ndim = self._device_data()[0].shape[1]
+        descs, jacs = zip(*[lower_jacobian(k, ndim) for k in kernels])
+        results = [(-np.inf, np.zeros(J.shape[1])) for J in jacs]
+        run, out = self._batched(indices, descs, backend.loglike_grad_batch, "tgp_loglike_grad_batch")
+        for i, o in zip(run, out if run else []):
+            results[i] = (float(o[0]), jacs[i].T @ o[3:3 + jacs[i].shape[0]])   # the gradient is 0 where logL = -inf
+        return results
+
     def solve(self):
-        """Fit every problem's kernel with the configured optimizer."""
+        """Fit every problem's kernel with the configured optimizer.  With log_likelihood.ANALYTIC_GRADIENT set (the
+        switch GPInterpolation honours), the "log-likelihood" searches use the analytic gradient: one batched
+        value-and-gradient call per round."""
         B = len(self._X)
         self._init_theta = [copy.deepcopy(k).theta for k in self.kernels]
         self._solved = None
-        if self.optimizer == "log-likelihood":
+        if self.optimizer == "log-likelihood" and log_likelihood.ANALYTIC_GRADIENT:
+            def evaluate_jac(indices, thetas):
+                vg = self._loglike_and_gradient(indices, [self.kernels[b].clone_with_theta(t)
+                                                          for b, t in zip(indices, thetas)])
+                return [(-v, -g) for v, g in vg]
+
+            best = lockstep_minimize(evaluate_jac, [k.theta for k in self.kernels], jac=True)
+            self.kernels = [self.kernels[b].clone_with_theta(best[b]) for b in range(B)]
+        elif self.optimizer == "log-likelihood":
             def evaluate(indices, thetas):
                 return -self._loglike(indices, [self.kernels[b].clone_with_theta(t) for b, t in zip(indices, thetas)])
 
