@@ -501,6 +501,11 @@ int tgp_pairbin_super_leaves(unsigned long long* host1 /*host*/, int reset);
  * in shared memory (the others went block by block, after a failed mirrored-bit check or when the staged tables do not
  * fit).  Synchronous. */
 int tgp_pairbin_super_rows(unsigned long long* host1 /*host*/, int reset);
+/* Diagnostics: how many super-chunk pairs with one varying axis (slot [6] of tgp_pairbin_stats) were decided per row
+ * point by the leaf kernel against the column super-chunk staged once for many such pairs.  The others were decided
+ * one at a time by the super kernel (when the staged tables do not fit, or "pairbin_fast_paths" lacks bit 1).  Not
+ * counted in tgp_pairbin_super_leaves or tgp_pairbin_super_rows.  Synchronous. */
+int tgp_pairbin_super_one_axis_rows(unsigned long long* host1 /*host*/, int reset);
 
 /* Test and measurement switches of the pair counts (tgp_pairbin_*, tgp_bootbin_twod), not needed for normal use.
  * Any other name is rejected with TGP_ERR_INVALID ("unknown option").

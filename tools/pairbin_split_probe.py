@@ -86,8 +86,9 @@ def worker(profile):
 
         count(c1, c1[5])
         backend.pairbin_stats(reset=True)
-        if hasattr(backend, "pairbin_super_leaves"):
-            backend.pairbin_super_leaves(reset=True)
+        for name in ("pairbin_super_leaves", "pairbin_super_rows", "pairbin_super_one_axis_rows"):
+            if hasattr(backend, name):
+                getattr(backend, name)(reset=True)
         torch.cuda.synchronize()
         with tprofile(activities=[ProfilerActivity.CUDA]) as prof:
             count(c1, c1[5])
@@ -100,6 +101,10 @@ def worker(profile):
         st = backend.pairbin_stats(reset=True)
         if hasattr(backend, "pairbin_super_leaves"):
             out["super_pairs_leaf_kernel"] = backend.pairbin_super_leaves(reset=True)
+        if hasattr(backend, "pairbin_super_rows"):
+            out["super_pairs_per_row"] = backend.pairbin_super_rows(reset=True)
+        if hasattr(backend, "pairbin_super_one_axis_rows"):
+            out["one_axis_super_pairs_leaf_kernel"] = backend.pairbin_super_one_axis_rows(reset=True)
         tot = sum(st.values())
         out["path_fractions"] = {k: v / tot for k, v in st.items()} if tot else st
     print("RESULT " + json.dumps(out), flush=True)

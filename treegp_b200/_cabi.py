@@ -111,6 +111,7 @@ SIGNATURES = {
     "tgp_pairbin_stats": [_vp, ctypes.c_int],
     "tgp_pairbin_super_leaves": [_vp, ctypes.c_int],
     "tgp_pairbin_super_rows": [_vp, ctypes.c_int],
+    "tgp_pairbin_super_one_axis_rows": [_vp, ctypes.c_int],
     "tgp_set_option": [ctypes.c_char_p, ctypes.c_int],
     "tgp_microbench_fp64": [ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)],
 }

@@ -928,6 +928,15 @@ def pairbin_super_rows(reset=True):
     return int(v.value)
 
 
+def pairbin_super_one_axis_rows(reset=True):
+    """Super-chunk pairs with one varying axis (pairbin_stats' super_one_axis, in super pairs) decided by the TwoD
+    leaf kernel against a column super-chunk staged for many of them (see tgp_pairbin_super_one_axis_rows)."""
+    v = ctypes.c_ulonglong(0)
+    check(_cabi.load().tgp_pairbin_super_one_axis_rows(ctypes.byref(v), int(bool(reset))),
+          "tgp_pairbin_super_one_axis_rows")
+    return int(v.value)
+
+
 def set_option(name, value):
     check(_cabi.load().tgp_set_option(name.encode(), int(value)), "tgp_set_option")
 

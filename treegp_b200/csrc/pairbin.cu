@@ -113,7 +113,9 @@ struct PBParams {
   int4* recs;
   int* rec_cnt;
   unsigned long long* counter_next;
-  unsigned long long* slist_len;   // super kernel / leaf kernel: length of the TWO_AXIS super pair list (pb_super_list)
+  unsigned long long* slist_len;   // super kernel / leaf kernel: length of the super pair list (pb_super_list)
+  int32_t list_one_axis;           // super kernel: ONE_AXIS super pairs are listed for the staged leaf kernel (1) or
+                                   // decided by the super kernel itself (0)
 };
 
 // Which path the pairs of all launches since the last reset took (in pairs): [0] closed form (block in one bin; TwoD:
@@ -1470,18 +1472,22 @@ __device__ __forceinline__ int pb_super_status(const double* __restrict__ srec, 
   return PB_S_TWO_AXIS;
 }
 
-// The list of TWO_AXIS super pairs follows the super records: {length, work counter of the leaf kernel} at `work` words
-// 3 and 4, entries {cat, R, C, x0 | y0 << 16} here, room for every super pair of every catalogue.
+// The list of super pairs for the leaf kernel follows the super records: {length, work counter of the leaf kernel} at
+// `work` words 3 and 4, entries {cat, R, C, x0 | y0 << 16} here, room for every super pair of every catalogue.  TWO_AXIS
+// entries carry the origin of their 2 x 2 window; ONE_AXIS entries (listed when the staged leaf kernel runs) carry
+// the two bins of pb_super_status with PB_E_ONE set and PB_E_VX set when x is the varying axis (nbins <= 4096 leaves
+// the top bits of each half free).
+constexpr int PB_E_ONE = 1 << 15, PB_E_VX = 1 << 14;
 __device__ __forceinline__ int4* pb_super_list(const PBParams& P) {
   return reinterpret_cast<int4*>(const_cast<double*>(pb_super_records(P)) +
                                  (size_t)PB_SUPER_STRIDE * (size_t)(P.cat_off[P.ncat] / PB_SUPER_PTS + P.ncat + 2));
 }
 
-// Super pairs per work item of the staged leaf kernel: a slice of the TWO_AXIS pairs that share a column super-chunk.
+// Super pairs per work item of the staged leaf kernel: a slice of the pairs of one kind that share a column super-chunk.
 // 128 measured best overall on a B200 (DESIGN section 5, v13): 256 builds fewer tables but balances worse at N = 2e5.
 constexpr int PB_LEAF_SLICE = 128;
-// Entries of the TWO_AXIS list (every super pair of every catalogue), super-chunk slots, and work items of the grouped
-// list (at most one partial slice per slot), from the total point count.
+// Entries of the list (every super pair of every catalogue), super-chunk slots, and work items of the grouped list (at
+// most one partial slice per slot and kind), from the total point count.
 __host__ __device__ __forceinline__ int64_t pb_super_list_cap(int64_t total) {
   const int64_t nsup = total / PB_SUPER_PTS;
   return nsup * (nsup > 0 ? nsup - 1 : 0) / 2;
@@ -1490,16 +1496,22 @@ __host__ __device__ __forceinline__ int64_t pb_super_slots(int64_t total, int32_
   return total / PB_SUPER_PTS + ncat + 2;
 }
 __host__ __device__ __forceinline__ int64_t pb_super_items_cap(int64_t total, int32_t ncat) {
-  return (pb_super_list_cap(total) / PB_LEAF_SLICE + pb_super_slots(total, ncat) + 1) & ~(int64_t)1;
+  return (pb_super_list_cap(total) / PB_LEAF_SLICE + 2 * pb_super_slots(total, ncat) + 1) & ~(int64_t)1;
 }
-// Behind the TWO_AXIS list: the links of the super-chunk records (PB_SUPER_PTS halfwords per slot: for every x-sorted
-// position, the point's index in the super-chunk | its position in the stored y-sorted copy << 8), one word per slot
-// (TWO_AXIS pairs with that column super-chunk, then their offset in the grouped list), the work items {first entry
-// << 16 | entries} and the list grouped by column super-chunk.  `boxes` = the chunk records.
+// Words per row of the DESCEND bitmap: one bit per super column of the longest catalogue, and more.
+__host__ __device__ __forceinline__ int64_t pb_super_desc_words(int64_t total) { return total / PB_SUPER_PTS / 32 + 1; }
+// Behind the list: the links of the super-chunk records (PB_SUPER_PTS halfwords per slot: for every x-sorted position,
+// the point's index in the super-chunk | its position in the stored y-sorted copy << 8), two words per slot (the
+// TWO_AXIS and the ONE_AXIS pairs with that column super-chunk, then their offsets in the grouped list), the work items
+// {first entry << 16 | entries}, the list grouped by column super-chunk and kind, and the DESCEND bitmap: bit C % 32 of
+// word desc[(slot of super row R) x pb_super_desc_words + C / 32] is set iff super pair (R, C) is DESCEND (written by
+// the super kernel for R < C < the catalogue's full super-chunks; one spare word at the end).  `boxes` = the chunk
+// records.
 struct PBSuperGroups {
   unsigned short* links;
   unsigned long long *goff, *items;
   int4* glist;
+  unsigned* desc;
 };
 __device__ __forceinline__ PBSuperGroups pb_super_groups(const double* boxes, const int64_t* cat_off, int32_t ncat) {
   const int64_t total = cat_off[ncat], nslot = pb_super_slots(total, ncat);
@@ -1508,9 +1520,66 @@ __device__ __forceinline__ PBSuperGroups pb_super_groups(const double* boxes, co
   g.links = reinterpret_cast<unsigned short*>(const_cast<int4*>(
       reinterpret_cast<const int4*>(rec + (size_t)PB_SUPER_STRIDE * (size_t)nslot) + pb_super_list_cap(total)));
   g.goff = reinterpret_cast<unsigned long long*>(g.links + (size_t)PB_SUPER_PTS * nslot);
-  g.items = g.goff + ((nslot + 1) & ~(int64_t)1);
+  g.items = g.goff + 2 * nslot;
   g.glist = reinterpret_cast<int4*>(g.items + pb_super_items_cap(total, ncat));
+  g.desc = reinterpret_cast<unsigned*>(g.glist + pb_super_list_cap(total));
   return g;
+}
+
+// One row point i of a ONE_AXIS super pair against the column super-chunk's copy sorted along the varying axis (sc:
+// PB_SUPER_PTS ascending coordinates, ss / sw: their suffix sums of k w and w), in shared memory.  pos = #{j : fl(c_j -
+// c_i) < t} by bisection with that predicate (monotone in c_j); the upper bin v0 + 1 gets PB_SUPER_PTS - pos pairs and
+// k_i w_i x suffix(pos) (w_i x suffix(pos)), added to up_c, up_s, up_w; the caller books the lower bin v0 as the rest.
+// The exact mirrored bits differ from the mirror image only for the columns between pos and pos_m = #{j : fl(c_j - c_i)
+// <= tm}, nearly always none; those pairs are moved in global memory (cb: the bin of the constant axis, vx: x varies).
+// Serves the staged leaf kernel and, where it does not run, the super kernel.
+template <bool WEIGHTED>
+__device__ __forceinline__ void pb_one_axis_row(const double* sc, const double* ss, const double* sw, double ci,
+                                                double ki, double wi, double t, double tm, int v0, int cb, bool vx,
+                                                int cat, const PBParams& P, unsigned& up_c, double& up_s,
+                                                double& up_w) {
+  const int nbins = P.nbins;
+  // pos = #{j : fl(c_j - c_i) < t} (branch-free lower bound over the ascending copy)
+  int pos = 0;
+#pragma unroll
+  for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
+    if (__dsub_rn(sc[pos + step - 1], ci) < t) pos += step;
+  if (pos == PB_SUPER_PTS - 1 && __dsub_rn(sc[pos], ci) < t) pos = PB_SUPER_PTS;
+  up_c += (unsigned)(PB_SUPER_PTS - pos);
+  const double sk = pos < PB_SUPER_PTS ? ss[pos] : 0.0;
+  up_s = fma(ki, sk, up_s);
+  double swp = 0.0;
+  if constexpr (WEIGHTED) { swp = pos < PB_SUPER_PTS ? sw[pos] : 0.0; up_w = fma(wi, swp, up_w); }
+  // exact mirrored bits: consistent iff pos_m == pos, i.e. column pos - 1 has the mirrored upper bit and column
+  // pos has not
+  const bool ok = (pos == 0 || __dsub_rn(sc[pos - 1], ci) <= tm) &&
+                  (pos == PB_SUPER_PTS || !(__dsub_rn(sc[pos], ci) <= tm));
+  if (!ok) {   // (rare) a column within rounding of a bin edge
+    int pm = 0;
+    for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
+      if (__dsub_rn(sc[pm + step - 1], ci) <= tm) pm += step;
+    if (pm == PB_SUPER_PTS - 1 && __dsub_rn(sc[pm], ci) <= tm) pm = PB_SUPER_PTS;
+    // columns [lo, hi) have a mirrored bin that is not the mirror image of their forward bin: pm > pos, forward
+    // upper bin whose mirrored entry is the upper mirrored bin; pm < pos, forward lower bin, mirrored lower bin
+    const int a = min(pos, pm), b = max(pos, pm);
+    const double kk = ki * ((a < PB_SUPER_PTS ? ss[a] : 0.0) - (b < PB_SUPER_PTS ? ss[b] : 0.0));
+    double ww = (double)(b - a);
+    if constexpr (WEIGHTED) ww = wi * ((a < PB_SUPER_PTS ? sw[a] : 0.0) - (b < PB_SUPER_PTS ? sw[b] : 0.0));
+    const int fv = pm > pos ? v0 + 1 : v0;                   // forward bin on the varying axis
+    const int av = nbins - 1 - fv;                           // assumed mirrored bin: the mirror image
+    const int xv = pm > pos ? nbins - 1 - v0 : nbins - 2 - v0;   // exact mirrored bin
+    const int mc = nbins - 1 - cb;                           // mirrored bin on the constant axis (exact)
+    const int assumed = vx ? mc * nbins + av : av * nbins + mc;
+    const int exact = vx ? mc * nbins + xv : xv * nbins + mc;
+    const size_t g = (size_t)cat * P.nb;
+    unsigned long long* cnt = reinterpret_cast<unsigned long long*>(P.npairs) + g;
+    atomicAdd(cnt + assumed, (unsigned long long)(-(long long)(b - a)));   // -(b - a) (mod 2^64)
+    atomicAdd(cnt + exact, (unsigned long long)(b - a));
+    atomicAdd(P.sumwkk + g + assumed, -kk);
+    atomicAdd(P.sumwkk + g + exact, kk);
+    atomicAdd(P.sumw + g + assumed, -ww);
+    atomicAdd(P.sumw + g + exact, ww);
+  }
 }
 template <bool WEIGHTED>
 __global__ void __launch_bounds__(PB_MAX_WARPS * 32, PB_CLASSIFY_MIN_CTAS)
@@ -1603,14 +1672,20 @@ pairbin_classify_kernel(PBParams P) {
       const int nlive = (it.ib == nblk - 1) ? tail : PB_CHUNK;
       int4* out = P.recs + (size_t)(q - P.q_begin) * (size_t)P.run;
       // the super kernel books or lists every super pair that is not DESCEND (on one rank); its blocks are skipped here
-      // on every rank.  Lane l decides super column cw + l; the chunks of the DESCEND ones are then classified 32 at a time.
-      const double* srec = pb_super_records(P) + (size_t)PB_SUPER_STRIDE * (size_t)(it.off / PB_SUPER_PTS + it.cat);
+      // on every rank.  Lane l takes super column cw + l (cw >= sR: c_lo >= ib), whose status the super kernel left in
+      // the DESCEND bitmap; the chunks of the DESCEND ones are then classified 32 at a time.
       const int64_t nsf = P.block_sums == 2 ? it.n / PB_SUPER_PTS : 0, sR = it.ib / PB_SUPER;
+      const unsigned* drow = nullptr;   // bitmap row of super row sR (rows at or past nsf are all DESCEND)
+      if (sR < nsf) {
+        const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
+        drow = grp.desc + (size_t)pb_super_desc_words(P.cat_off[P.ncat]) * (size_t)(it.off / PB_SUPER_PTS + it.cat + sR);
+      }
       for (int64_t cw = it.c_lo / PB_SUPER; cw * PB_SUPER < it.c_hi; cw += 32) {
-        int sx0, sy0;
-        bool svx;
-        const unsigned dm = __ballot_sync(0xffffffffu, (cw + lane) * PB_SUPER < it.c_hi &&
-            pb_super_status(srec, nsf, sR, cw + lane, M, lo2, nbins, ed, sx0, sy0, svx) == PB_S_DESCEND);
+        unsigned bits = ~0u;   // the 32 bits from super column cw on
+        if (drow) bits = __funnelshift_r(drow[cw >> 5], drow[(cw >> 5) + 1], (unsigned)(cw & 31));
+        const int64_t C = cw + lane;
+        const unsigned dm = __ballot_sync(0xffffffffu, C * PB_SUPER < it.c_hi &&
+                                                           (C <= sR || C >= nsf || ((bits >> lane) & 1u)));
         const int nd = __popc(dm) * PB_SUPER;
         const int base = (int)(cw * PB_SUPER - it.c_lo);   // negative only for the diagonal super-chunk
         for (int s0 = 0; s0 < nd; s0 += 32) {
@@ -1759,7 +1834,7 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
   {
     unsigned long long* goff = pb_super_groups(boxes, cat_off, ncat).goff;
     const int64_t nslot = pb_super_slots(cat_off[ncat], ncat);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + t; i < nslot; i += (int64_t)gridDim.x * blockDim.x)
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + t; i < 2 * nslot; i += (int64_t)gridDim.x * blockDim.x)
       goff[i] = 0ull;
   }
   const int64_t cat = blockIdx.x / supers_per_cat, s = blockIdx.x % supers_per_cat;
@@ -1822,15 +1897,15 @@ pairbin_super_boxes_kernel(const double* __restrict__ px, const double* __restri
   }
 }
 
-// The super kernel: books every super pair that is not DESCEND, once per count, before the rounds.  Items are (super
-// row R, run of 32 super columns) of this rank, dealt like the chunk items; lane l takes the status of super pair
-// (R, 32 r + l).
+// The super kernel: decides the status of every super pair once per count, before the rounds, and books or lists every
+// one that is not DESCEND.  Items are (super row R, run of 32 super columns); lane l takes the status of super pair
+// (R, 32 r + l), and the warp writes the run's word of the DESCEND bitmap that the classification pass reads.  Every
+// rank sweeps all items (the classification pass of a rank reads super pairs of every item); the items q with
+// q % nranks == rank are its own:
 //   CLOSED    booked by its lane: count n_R n_C, sum (sum k w)_R (sum k w)_C (forward entry only);
-//   ONE_AXIS  one pair at a time by the warp: the column super-chunk's copy sorted along the varying axis is staged in
-//             shared memory, and every row point i finds pos = #{j : fl(c_j - c_i) < t} by bisection with that
-//             predicate (monotone in c_j).  The upper bin gets n_C - pos pairs and k_i w_i x suffix(pos), the lower bin
-//             the rest.  The exact mirrored bits differ from the mirror image only for the columns between pos and
-//             pos_m = #{j : fl(c_j - c_i) <= -t_m}, nearly always none; those pairs are moved in global memory.
+//   ONE_AXIS  with list_one_axis: appended to the list of the staged leaf kernel like TWO_AXIS.  Otherwise one pair at a
+//             time by the warp: the column super-chunk's copy sorted along the varying axis is staged in shared memory
+//             and every row point takes pb_one_axis_row; the lower bin gets the rest of the pairs and sums;
 //   TWO_AXIS  appended to the list of the leaf kernel (pairbin_super_leaves_kernel) and counted per column super-chunk.
 // The warp histograms hold forward entries; the mirror image is added when they are written out.
 template <bool WEIGHTED>
@@ -1885,6 +1960,8 @@ pairbin_super_kernel(PBParams P) {
   const double* sup0 = pb_super_records(P);
   int4* slist = pb_super_list(P);
   unsigned long long* goff = pb_super_groups(P.boxes, P.cat_off, P.ncat).goff;
+  unsigned* desc = pb_super_groups(P.boxes, P.cat_off, P.ncat).desc;
+  const int64_t dwords = pb_super_desc_words(P.cat_off[P.ncat]);
   const int64_t nruns = (P.items_per_cat + 31) / 32;   // items_per_cat: super-chunks of the longest catalogue
   unsigned st_closed = 0, st_one = 0;   // super pairs
   int cur_cat = -1, since_flush = 0;
@@ -1893,34 +1970,42 @@ pairbin_super_kernel(PBParams P) {
     if (lane == 0) q = atomicAdd(P.counter, 1ull);
     q = __shfl_sync(0xffffffffu, q, 0);
     if ((int64_t)q >= P.my_items) break;
-    const int64_t item = (int64_t)q * P.nranks + P.rank;
+    // every rank sweeps the status of every super pair into the DESCEND bitmap (its classification pass reads super
+    // pairs of every item); it books and lists only the items dealt to it
+    const int64_t item = (int64_t)q;
+    const bool mine = (int64_t)(q % (unsigned long long)P.nranks) == P.rank;
     const int cat = (int)(item / (P.items_per_cat * nruns));
     if (cat >= P.ncat) break;
     const int64_t R = (item % (P.items_per_cat * nruns)) / nruns, r = item % nruns;
     const int64_t off = P.cat_off[cat], n = P.cat_off[cat + 1] - off;
     const int64_t nsf = n / PB_SUPER_PTS;
     if (R >= nsf || (r + 1) * 32 <= R + 1 || r * 32 >= nsf) continue;   // no super column C > R in this run
+    const double* srec = sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat);
+    const int64_t C = r * 32 + lane;
+    int x0 = 0, y0 = 0;
+    bool vx = false;
+    const int st = C > R ? pb_super_status(srec, nsf, R, C, M, lo2, nbins, ed, x0, y0, vx) : PB_S_DESCEND;
+    const unsigned dsc = __ballot_sync(0xffffffffu, st == PB_S_DESCEND);
+    if (lane == 0) desc[(size_t)dwords * (size_t)(off / PB_SUPER_PTS + cat + R) + r] = dsc;
+    if (!mine) continue;
     if (cat != cur_cat || since_flush >= PB_SUPER_FLUSH_ITEMS) {
       flush_hist(cur_cat);
       cur_cat = cat;
       since_flush = 0;
     }
     ++since_flush;
-    const double* srec = sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat);
-    const double* rrec = srec + (size_t)PB_SUPER_STRIDE * (size_t)R;
-    const double2 rsum = *reinterpret_cast<const double2*>(rrec + 4);
-    const int64_t C = r * 32 + lane;
-    int x0 = 0, y0 = 0;
-    bool vx = false;
-    const int st = C > R ? pb_super_status(srec, nsf, R, C, M, lo2, nbins, ed, x0, y0, vx) : PB_S_DESCEND;
-    const unsigned two = __ballot_sync(0xffffffffu, st == PB_S_TWO_AXIS);
-    if (two) {   // appended for the leaf kernel: one atomic per warp step
+    const double2 rsum = *reinterpret_cast<const double2*>(srec + (size_t)PB_SUPER_STRIDE * (size_t)R + 4);
+    const bool one = st == PB_S_ONE_AXIS;
+    const bool listed = st == PB_S_TWO_AXIS || (one && P.list_one_axis);
+    const unsigned lst = __ballot_sync(0xffffffffu, listed);
+    if (lst) {   // appended for the leaf kernel: one atomic per warp step
       unsigned long long base = 0;
-      if (lane == 0) base = atomicAdd(P.slist_len, (unsigned long long)__popc(two));
+      if (lane == 0) base = atomicAdd(P.slist_len, (unsigned long long)__popc(lst));
       base = __shfl_sync(0xffffffffu, base, 0);
-      if (st == PB_S_TWO_AXIS) {
-        slist[base + __popc(two & ((1u << lane) - 1u))] = make_int4(cat, (int)R, (int)C, x0 | (y0 << 16));
-        atomicAdd(goff + off / PB_SUPER_PTS + cat + C, 1ull);   // group size of column super-chunk C
+      if (listed) {
+        const int ew = one ? x0 | (y0 << 16) | PB_E_ONE | (vx ? PB_E_VX : 0) : x0 | (y0 << 16);
+        slist[base + __popc(lst & ((1u << lane) - 1u))] = make_int4(cat, (int)R, (int)C, ew);
+        atomicAdd(goff + 2 * (off / PB_SUPER_PTS + cat + C) + (one ? 1 : 0), 1ull);   // group size of (C, kind)
       }
     }
     if (st == PB_S_CLOSED) {
@@ -1931,7 +2016,7 @@ pairbin_super_kernel(PBParams P) {
       if constexpr (WEIGHTED) atomicAdd(my_w + o, rsum.y * csum.y);
       ++st_closed;
     }
-    unsigned todo = __ballot_sync(0xffffffffu, st == PB_S_ONE_AXIS);
+    unsigned todo = __ballot_sync(0xffffffffu, one && !P.list_one_axis);
     while (todo) {
       const int c = __ffs(todo) - 1;
       todo &= todo - 1;
@@ -1959,48 +2044,7 @@ pairbin_super_kernel(PBParams P) {
         const double ci = rc[i];
         double wi = 1.0;
         if constexpr (WEIGHTED) wi = rw[i];
-        const double ki = rk[i] * wi;
-        // pos = #{j : fl(c_j - c_i) < t} (branch-free lower bound over the ascending copy)
-        int pos = 0;
-#pragma unroll
-        for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
-          if (__dsub_rn(sc[pos + step - 1], ci) < t) pos += step;
-        if (pos == PB_SUPER_PTS - 1 && __dsub_rn(sc[pos], ci) < t) pos = PB_SUPER_PTS;
-        up_c += (unsigned)(PB_SUPER_PTS - pos);
-        const double sk = pos < PB_SUPER_PTS ? ss[pos] : 0.0;
-        up_s = fma(ki, sk, up_s);
-        double swp = 0.0;
-        if constexpr (WEIGHTED) { swp = pos < PB_SUPER_PTS ? sw[pos] : 0.0; up_w = fma(wi, swp, up_w); }
-        // exact mirrored bits: consistent iff pos_m == pos, i.e. column pos - 1 has the mirrored upper bit and column
-        // pos has not
-        const bool ok = (pos == 0 || __dsub_rn(sc[pos - 1], ci) <= tm) &&
-                        (pos == PB_SUPER_PTS || !(__dsub_rn(sc[pos], ci) <= tm));
-        if (!ok) {   // (rare) a column within rounding of a bin edge
-          int pm = 0;
-          for (int step = PB_SUPER_PTS / 2; step >= 1; step >>= 1)
-            if (__dsub_rn(sc[pm + step - 1], ci) <= tm) pm += step;
-          if (pm == PB_SUPER_PTS - 1 && __dsub_rn(sc[pm], ci) <= tm) pm = PB_SUPER_PTS;
-          // columns [lo, hi) have a mirrored bin that is not the mirror image of their forward bin: pm > pos, forward
-          // upper bin whose mirrored entry is the upper mirrored bin; pm < pos, forward lower bin, mirrored lower bin
-          const int a = min(pos, pm), b = max(pos, pm);
-          const double kk = ki * ((a < PB_SUPER_PTS ? ss[a] : 0.0) - (b < PB_SUPER_PTS ? ss[b] : 0.0));
-          double ww = (double)(b - a);
-          if constexpr (WEIGHTED) ww = wi * ((a < PB_SUPER_PTS ? sw[a] : 0.0) - (b < PB_SUPER_PTS ? sw[b] : 0.0));
-          const int fv = pm > pos ? v0 + 1 : v0;                   // forward bin on the varying axis
-          const int av = nbins - 1 - fv;                           // assumed mirrored bin: the mirror image
-          const int xv = pm > pos ? nbins - 1 - v0 : nbins - 2 - v0;   // exact mirrored bin
-          const int mc = nbins - 1 - cb;                           // mirrored bin on the constant axis (exact)
-          const int assumed = cvx ? mc * nbins + av : av * nbins + mc;
-          const int exact = cvx ? mc * nbins + xv : xv * nbins + mc;
-          const size_t g = (size_t)cat * nb;
-          unsigned long long* cnt = reinterpret_cast<unsigned long long*>(P.npairs) + g;
-          atomicAdd(cnt + assumed, (unsigned long long)(-(long long)(b - a)));   // -(b - a) (mod 2^64)
-          atomicAdd(cnt + exact, (unsigned long long)(b - a));
-          atomicAdd(P.sumwkk + g + assumed, -kk);
-          atomicAdd(P.sumwkk + g + exact, kk);
-          atomicAdd(P.sumw + g + assumed, -ww);
-          atomicAdd(P.sumw + g + exact, ww);
-        }
+        pb_one_axis_row<WEIGHTED>(sc, ss, sw, ci, rk[i] * wi, wi, t, tm, v0, cb, cvx, cat, P, up_c, up_s, up_w);
       }
       up_c = warp_sum_u(up_c);
       up_s = warp_sum(up_s);
@@ -2030,15 +2074,19 @@ pairbin_super_kernel(PBParams P) {
 // point against the staged column super-chunk (tgp_pairbin_super_rows).  Diagnostics.
 __device__ unsigned long long g_pb_super_leaves;
 __device__ unsigned long long g_pb_super_rows;
+// ONE_AXIS super pairs decided by the staged leaf kernel since the last reset (tgp_pairbin_super_one_axis_rows): those
+// not counted here were decided by the super kernel.  Diagnostics.
+__device__ unsigned long long g_pb_super_one_rows;
 
-// Grouping of the TWO_AXIS list by column super-chunk, for the staged leaf kernel (one CTA): the group sizes counted by
-// the super kernel become offsets (exclusive scan over the slots), and every group is cut into work items of at most
-// PB_LEAF_SLICE entries.  The number of items goes to work word 5 (P.slist_len[2]); the host never reads it.
+// Grouping of the list by column super-chunk and kind, for the staged leaf kernel (one CTA): the group sizes counted by
+// the super kernel (two per slot: TWO_AXIS, ONE_AXIS) become offsets (exclusive scan over the groups), and every group
+// is cut into work items of at most PB_LEAF_SLICE entries, so that an item holds one kind only.  The number of items
+// goes to work word 5 (P.slist_len[2]); the host never reads it.
 __global__ void __launch_bounds__(1024) pairbin_super_group_kernel(PBParams P) {
   __shared__ unsigned long long s_part[2][32];
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
-  const int64_t nslot = pb_super_slots(P.cat_off[P.ncat], P.ncat);
+  const int64_t nslot = 2 * pb_super_slots(P.cat_off[P.ncat], P.ncat);   // groups
   const int64_t per = (nslot + blockDim.x - 1) / blockDim.x;
   const int64_t s0 = min((int64_t)t * per, nslot), s1 = min(s0 + per, nslot);
   unsigned long long c = 0, m = 0;
@@ -2067,7 +2115,7 @@ __global__ void __launch_bounds__(1024) pairbin_super_group_kernel(PBParams P) {
   if (t == (int)blockDim.x - 1) P.slist_len[2] = io;
 }
 
-// Scatter of the TWO_AXIS list into its groups (the order inside a group is immaterial).
+// Scatter of the list into its groups (the order inside a group is immaterial).
 __global__ void __launch_bounds__(256) pairbin_super_scatter_kernel(PBParams P) {
   const PBSuperGroups grp = pb_super_groups(P.boxes, P.cat_off, P.ncat);
   const int4* slist = pb_super_list(P);
@@ -2075,7 +2123,8 @@ __global__ void __launch_bounds__(256) pairbin_super_scatter_kernel(PBParams P) 
   for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
        i += (unsigned long long)gridDim.x * blockDim.x) {
     const int4 e = slist[i];
-    grp.glist[atomicAdd(grp.goff + P.cat_off[e.x] / PB_SUPER_PTS + e.x + e.z, 1ull)] = e;
+    const int64_t g = 2 * (P.cat_off[e.x] / PB_SUPER_PTS + e.x + e.z) + ((e.w & PB_E_ONE) ? 1 : 0);
+    grp.glist[atomicAdd(grp.goff + g, 1ull)] = e;
   }
 }
 
@@ -2181,8 +2230,11 @@ struct PBLeafTable {
 // Each axis has one bit per pair, fixed per super pair (pb_leaf_bits).
 //
 // STAGED (the default when the tables fit in shared memory): work items are slices of the list grouped by column
-// super-chunk C (pairbin_super_group_kernel).  A CTA claims an item, stages C's sorted copies and the dominance table
-// (PBLeafTable) once, and its warps pull the slice's super pairs from a shared counter.  For each of the 256 row points
+// super-chunk C and kind (pairbin_super_group_kernel).  A CTA claims an item, stages C's sorted copies and, for a
+// TWO_AXIS item, the dominance table (PBLeafTable) once, and its warps pull the slice's super pairs from a shared
+// counter.  A ONE_AXIS super pair (the list holds them only in this form) takes pb_one_axis_row for each of its 256
+// row points against the staged copy of its varying axis, and is booked like a TWO_AXIS pair; it needs no table and
+// no per-block body, and its pairs go to path statistic [6] as the super kernel's did.  For each of the 256 row points
 // of a super pair, p_x and p_y come from bisections on the staged copies and the four sums from the suffix sums and the
 // table; the exact mirrored bits need only the neighbours of each split.  If any check fails (a column within rounding
 // of a bin edge), the super pair goes through the per-block body below instead.  One histogram per CTA, booked with
@@ -2292,7 +2344,7 @@ pairbin_super_leaves_kernel(PBParams P) {
 
   const double M = P.hi, lo2 = P.lo2;
   const double* sup0 = pb_super_records(P);
-  unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0, st_rows = 0;
+  unsigned st_closed = 0, st_1d = 0, st_pw = 0, st_sorted = 0, st_quad = 0, st_pairs = 0, st_rows = 0, st_one = 0;
 
   // ---- one super pair (one warp) ----
   auto decide = [&](const int4 e) {
@@ -2611,6 +2663,56 @@ pairbin_super_leaves_kernel(PBParams P) {
     __syncwarp();
   };
 
+  // ---- one ONE_AXIS super pair (one warp, STAGED): per row point against the staged copy of the varying axis ----
+  auto decide_one = [&](const int4 e) {
+    const int cat = e.x, x0 = e.w & 0xfff, y0 = (e.w >> 16) & 0xfff;
+    const bool vx = (e.w & PB_E_VX) != 0;
+    const int v0 = vx ? x0 : y0, cb = vx ? y0 : x0;   // varying axis: bins v0, v0 + 1; constant axis: bin cb
+    const double t = ed[v0 + 1], tm = -ed[nbins - 1 - v0];   // forward upper bit: d >= t; mirrored upper bit: d <= tm
+    const int64_t off = P.cat_off[cat];
+    const int64_t rb = off + (int64_t)e.y * PB_SUPER_PTS + lane;
+    const double* rc = vx ? P.px : P.py;
+    const double *sc = vx ? T.xs : T.ys, *ss = vx ? T.sxk : T.syk, *sw = vx ? T.sxw : T.syw;
+    double up_s = 0.0, up_w = 0.0;
+    unsigned up_c = 0u;
+    // four row points at a time: their loads issued together, then four independent bisections (the pair is bound by
+    // the latency of the loads and of the dependent probes, not by their number)
+#pragma unroll 1
+    for (int h = 0; h < PB_SUPER; h += 4) {
+      double ci[4], ki[4], wi[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const int64_t i = rb + (h + k) * 32;
+        ci[k] = rc[i];
+        wi[k] = 1.0;
+        if constexpr (WEIGHTED) wi[k] = P.pw[i];
+        ki[k] = P.pk[i];
+      }
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        pb_one_axis_row<WEIGHTED>(sc, ss, sw, ci[k], ki[k] * wi[k], wi[k], t, tm, v0, cb, vx, cat, P, up_c, up_s, up_w);
+    }
+    up_c = warp_sum_u(up_c);
+    up_s = warp_sum(up_s);
+    if constexpr (WEIGHTED) up_w = warp_sum(up_w);
+    if (lane == 0) {   // the CTA histogram (forward entries)
+      const double2 rsum = *reinterpret_cast<const double2*>(
+          sup0 + (size_t)PB_SUPER_STRIDE * (size_t)(off / PB_SUPER_PTS + cat + e.y) + 4);
+      const int lo_b = vx ? cb * nbins + v0 : v0 * nbins + cb;
+      const int hi_b = vx ? cb * nbins + v0 + 1 : (v0 + 1) * nbins + cb;
+      atomicAdd(hc_cta + lo_b, (unsigned long long)((unsigned)(PB_SUPER_PTS * PB_SUPER_PTS) - up_c));
+      atomicAdd(my_s + lo_b, rsum.x * T.sxk[0] - up_s);
+      atomicAdd(hc_cta + hi_b, (unsigned long long)up_c);
+      atomicAdd(my_s + hi_b, up_s);
+      if constexpr (WEIGHTED) {
+        atomicAdd(my_w + lo_b, rsum.y * T.sxw[0] - up_w);
+        atomicAdd(my_w + hi_b, up_w);
+      }
+    }
+    ++st_one;
+    __syncwarp();
+  };
+
   if constexpr (STAGED) {
     __shared__ unsigned long long s_item;
     __shared__ unsigned s_next;
@@ -2636,7 +2738,9 @@ pairbin_super_leaves_kernel(PBParams P) {
         flush_cta(cur_cat);
         cur_cat = e0.x;
       }
-      // ---- stage column super-chunk C: sorted copies, suffix sums, k w and w in x order, the links ----
+      // ---- stage column super-chunk C: sorted copies, suffix sums; for TWO_AXIS items also k w and w in x order and
+      // the links.  An item holds one kind only; ONE_AXIS items need no dominance table ----
+      const bool one_item = (e0.w & PB_E_ONE) != 0;
       {
         const int64_t off = P.cat_off[e0.x], slot = off / PB_SUPER_PTS + e0.x + e0.z;
         const double* crec = sup0 + (size_t)PB_SUPER_STRIDE * (size_t)slot + PB_SLOT;
@@ -2647,12 +2751,15 @@ pairbin_super_leaves_kernel(PBParams P) {
           T.sxk[i] = crec[SP + i];
           T.ys[i] = crec[3 * SP + i];
           T.syk[i] = crec[4 * SP + i];
+          if constexpr (WEIGHTED) {
+            T.sxw[i] = crec[2 * SP + i];
+            T.syw[i] = crec[5 * SP + i];
+          }
+          if (one_item) continue;
           const unsigned l = lk[i];
           const int j = (int)(l & 0xffu), r = (int)(l >> 8);
           double wj = 1.0;
           if constexpr (WEIGHTED) {
-            T.sxw[i] = crec[2 * SP + i];
-            T.syw[i] = crec[5 * SP + i];
             wj = P.pw[base + j];
             T.wx[i] = wj;
           }
@@ -2665,13 +2772,23 @@ pairbin_super_leaves_kernel(PBParams P) {
           T.syk[SP] = 0.0;
           if constexpr (WEIGHTED) { T.sxw[SP] = 0.0; T.syw[SP] = 0.0; }
         }
-        for (int i = tid; i < N; i += nthr) {   // row NB of U: no x-block
+        for (int i = tid; i < N && !one_item; i += nthr) {   // row NB of U: no x-block
           T.uk[PB_LT_NB * N + i] = 0.0;
           T.uc[PB_LT_NB * N + i] = 0;
           if constexpr (WEIGHTED) T.uw[PB_LT_NB * N + i] = 0.0;
         }
       }
       __syncthreads();
+      if (one_item) {   // ---- the slice's ONE_AXIS super pairs, one per warp step ----
+        while (true) {
+          unsigned k = 0;
+          if (lane == 0) k = atomicAdd(&s_next, 1u);
+          k = __shfl_sync(0xffffffffu, k, 0);
+          if ((int)k >= len) break;
+          decide_one(slice[k]);
+        }
+        continue;
+      }
       // in-block y order of every x position; U row by row (one warp per x-block: suffix scans over the y order)
       for (int p = tid; p < SP; p += nthr) {
         const int b0 = p & ~(XB - 1), r = T.yr[p];
@@ -2769,6 +2886,10 @@ pairbin_super_leaves_kernel(PBParams P) {
     if (st_quad) atomicAdd(&g_pb_stats[4], LEAF * st_quad);
     if (st_pairs) atomicAdd(&g_pb_super_leaves, (unsigned long long)st_pairs);
     if (st_rows) atomicAdd(&g_pb_super_rows, (unsigned long long)st_rows);
+    if (st_one) {
+      atomicAdd(&g_pb_stats[6], (unsigned long long)PB_SUPER_PTS * PB_SUPER_PTS * st_one);
+      atomicAdd(&g_pb_super_one_rows, (unsigned long long)st_one);
+    }
   }
 }
 
@@ -2793,7 +2914,7 @@ static int64_t pb_rec_slots(int64_t max_len, int32_t ncat) {
 }
 // Work buffer of the two-pass count: {work counters of pass A, pass B, the super kernel; length of the TWO_AXIS list,
 // work counter of the leaf kernel, its number of work items; 2 spare words} {record counts of a round: slots / 32 ints}
-// {records: 2 doubles each} {pre-pass chunk records} {super-chunk records} {TWO_AXIS list: 2 doubles per super pair}
+// {records: 2 doubles each} {pre-pass chunk records} {super-chunk records} {super pair list: 2 doubles per super pair}
 // {the regions of pb_super_groups}.  The other paths keep the chunk records at the start.
 static int64_t pb_rec_region_doubles(int64_t slots) { return 8 + slots / 64 + 2 * slots; }
 
@@ -2801,8 +2922,8 @@ extern "C" int64_t tgp_pairbin_work_doubles(int64_t total_points, int32_t ncat) 
   const int64_t nslot = pb_super_slots(total_points, ncat);
   return pb_rec_region_doubles(pb_rec_slots(total_points, ncat)) +
          (int64_t)PB_STRIDE * (total_points / PB_CHUNK + (int64_t)ncat + 2) + (int64_t)PB_SUPER_STRIDE * nslot +
-         4 * pb_super_list_cap(total_points) + (int64_t)PB_SUPER_PTS / 4 * nslot + ((nslot + 1) & ~(int64_t)1) +
-         pb_super_items_cap(total_points, ncat);
+         4 * pb_super_list_cap(total_points) + (int64_t)PB_SUPER_PTS / 4 * nslot + 2 * nslot +
+         pb_super_items_cap(total_points, ncat) + (nslot * pb_super_desc_words(total_points) + 2) / 2;
 }
 
 static int g_pb_fast_paths = 7;   // tgp_set_option("pairbin_fast_paths", bits): see PBParams::fast_paths
@@ -2826,6 +2947,16 @@ extern "C" int tgp_pairbin_super_rows(unsigned long long* host1, int reset) {
   if (reset) {
     const unsigned long long z = 0;
     TGP_CUDA(cudaMemcpyToSymbol(g_pb_super_rows, &z, sizeof(z)));
+  }
+  return TGP_OK;
+}
+
+extern "C" int tgp_pairbin_super_one_axis_rows(unsigned long long* host1, int reset) {
+  TGP_CHECK_ARG(host1 != nullptr, "host1");
+  TGP_CUDA(cudaMemcpyFromSymbol(host1, g_pb_super_one_rows, sizeof(unsigned long long)));
+  if (reset) {
+    const unsigned long long z = 0;
+    TGP_CUDA(cudaMemcpyToSymbol(g_pb_super_one_rows, &z, sizeof(z)));
   }
   return TGP_OK;
 }
@@ -2928,6 +3059,7 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
   P.rec_cnt = nullptr;
   P.counter_next = nullptr;
   P.slist_len = nullptr;
+  P.list_one_axis = 0;
   if (work) {
     TGP_CHECK_ARG(((uintptr_t)work % 32) == 0, "work must be 32-byte aligned");
     double* bx = work + (split ? pb_rec_region_doubles(rec_slots) : 0);
@@ -2956,13 +3088,33 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
     int warps_s = (int)((budget - fixed - 64) / per_warp_s);
     if (warps_s > PB_MAX_WARPS) warps_s = PB_MAX_WARPS;
     const bool supers = nsf_max >= 2 && warps_s >= 1;
+    // the leaf kernel takes the super pairs the super kernel listed (the length stays on the device).  Staged (the
+    // per-row form of the 2 x 2 window is on): the list grouped by column super-chunk and kind, the tables of one
+    // super-chunk + a CTA histogram + one staged column chunk per warp, 2 CTAs of 8 warps per SM, or one of 16 if only
+    // that fits; the ONE_AXIS super pairs are listed too.  Otherwise warp histograms + one staged column chunk per
+    // warp, and the super kernel decides the ONE_AXIS super pairs itself.
+    const size_t hist_t = (size_t)P.nb * (8 + 8 + (weighted ? 8 : 0));
+    auto smem_t = [&](int w) {
+      return fixed + (size_t)w * PB_CHUNK * (16 + 8 + 8) + hist_t + pb_leaf_table_bytes(weighted) + 64;
+    };
+    // what one CTA takes of the SM's 228 KB: dynamic + static shared memory (the item and pair claims) + the 1 KB the
+    // driver reserves per CTA, in 128-byte allocation units
+    auto cta_t = [&](int w) { return (smem_t(w) + 16 + 1024 + 127) / 128 * 128; };
+    int warps_t = 0, ctas_t = 0;
+    if (P.fast_paths & 2) {
+      if (2 * cta_t(PB_MAX_WARPS) <= 228 * 1024) { warps_t = PB_MAX_WARPS; ctas_t = 2; }
+      else if (smem_t(2 * PB_MAX_WARPS) <= 226 * 1024) { warps_t = 2 * PB_MAX_WARPS; ctas_t = 1; }
+    }
     PBParams PS = P;
     const int64_t super_items = nsf_max * ((nsf_max + 31) / 32) * ncat;
     PS.items_per_cat = nsf_max;   // the super kernel's items of a catalogue: nsf_max rows x runs of 32 columns
-    PS.my_items = (super_items - tile_rank + tile_nranks - 1) / tile_nranks;
+    // every rank sweeps the statuses of all items (the DESCEND bitmap of its classification pass) and books or lists
+    // those with item % nranks == rank
+    PS.my_items = super_items;
     PS.counter = ctr + 2;
     PS.slist_len = ctr + 3;
     PS.warps = warps_s;
+    PS.list_one_axis = warps_t ? 1 : 0;
     const size_t smem_s = fixed + (size_t)warps_s * per_warp_s + 64;
     if (supers) {
       pairbin_super_boxes_kernel<<<(unsigned)(nsf_max * ncat), PB_SUPER_PTS, 0, st>>>(
@@ -2983,26 +3135,10 @@ extern "C" int tgp_pairbin(const double* px, const double* py, const double* pk,
       if (weighted) pairbin_super_kernel<true><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
       else pairbin_super_kernel<false><<<(unsigned)grid_s, warps_s * 32, smem_s, st>>>(PS);
       TGP_LAUNCH_CHECK();
-      // the leaf kernel takes the TWO_AXIS super pairs the super kernel listed (the length stays on the device).
-      // Staged (the per-row form of the 2 x 2 window is on): the list grouped by column super-chunk, the tables of one
-      // super-chunk + a CTA histogram + one staged column chunk per warp, 2 CTAs of 8 warps per SM, or one of 16 if
-      // only that fits.  Otherwise warp histograms + one staged column chunk per warp; per_warp_l < per_warp_s, so
-      // warps_l >= 1.
+      // the leaf kernel (per_warp_l < per_warp_s, so warps_l >= 1 when it is not staged)
       PBParams PL = P;
       PL.counter = ctr + 4;
       PL.slist_len = ctr + 3;
-      const size_t hist_t = (size_t)P.nb * (8 + 8 + (weighted ? 8 : 0));
-      auto smem_t = [&](int w) {
-        return fixed + (size_t)w * PB_CHUNK * (16 + 8 + 8) + hist_t + pb_leaf_table_bytes(weighted) + 64;
-      };
-      // what one CTA takes of the SM's 228 KB: dynamic + static shared memory (the item and pair claims) + the 1 KB the
-      // driver reserves per CTA, in 128-byte allocation units
-      auto cta_t = [&](int w) { return (smem_t(w) + 16 + 1024 + 127) / 128 * 128; };
-      int warps_t = 0, ctas_t = 0;
-      if (P.fast_paths & 2) {
-        if (2 * cta_t(PB_MAX_WARPS) <= 228 * 1024) { warps_t = PB_MAX_WARPS; ctas_t = 2; }
-        else if (smem_t(2 * PB_MAX_WARPS) <= 226 * 1024) { warps_t = 2 * PB_MAX_WARPS; ctas_t = 1; }
-      }
       if (warps_t) {
         pairbin_super_group_kernel<<<1, 1024, 0, st>>>(PL);
         TGP_LAUNCH_CHECK();
