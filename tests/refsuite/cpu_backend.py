@@ -95,17 +95,20 @@ def install():
     def loglike(X, y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
         X = backend.as_points(X)
         n = X.shape[0]
-        work = backend.alloc_matrix(n + 1, n) if work is None else work
+        Y = _np(y)
+        cols = [Y] if Y.ndim == 1 else [Y[:, c] for c in range(Y.shape[1])]   # y (n,) or (n, r): the joint logL
+        work = backend.alloc_matrix(n + len(cols), n) if work is None else work
         K = _kmat(kdesc, X) + np.diag(_np(yerr2))
-        logl, alpha = go.log_likelihood(K, _np(y))
+        fits = [go.log_likelihood(K, c) for c in cols]
         info = torch.zeros(1, dtype=torch.int32)
         out = torch.zeros(3, dtype=F64)
-        if alpha is None:
+        if fits[0][1] is None:
             info[0] = 1
             out[0] = -np.inf
-            alpha = np.zeros(n)
+            alpha = np.zeros(Y.shape)
         else:
-            out[0] = logl
+            out[0] = sum(logl for logl, _ in fits)
+            alpha = fits[0][1] if Y.ndim == 1 else np.stack([a for _, a in fits], axis=1)
             il = np.tril_indices(n)
             _np(work)[:n, :n][il] = sla.cholesky(K, lower=True)[il]   # the factor stays in the workspace
         return out, info, torch.as_tensor(alpha), work

@@ -49,7 +49,7 @@ def _sorted(X, desc, Y, e2):
 
 @pytest.mark.parametrize("r", [1, 2, 3, 8])
 @pytest.mark.parametrize("case", list(CASES) + list(CASES_1D))
-def test_multi_entries_against_single_output_runs(gpu_ready, case, r):
+def test_outputs_as_columns_against_single_output_runs(gpu_ready, case, r):
     """Each column of alpha (K^-1 Y and L^-1 Y) and of the truncated mean is its single-output run bit for bit; the
     joint logL and gradient are the sums of the single-output ones; with r = 1 everything is bit for bit."""
     from treegp_b200 import backend
@@ -62,7 +62,7 @@ def test_multi_entries_against_single_output_runs(gpu_ready, case, r):
     Xs = backend.as_points(np.random.default_rng(9).uniform(0, field, size=(20000, ndim)))
     for re in (None, row_end):
         for want_alpha in (False, True):
-            out, info, alpha, _ = backend.loglike_multi(Xo, Yo, eo, d, want_alpha=want_alpha, row_end=re)
+            out, info, alpha, _ = backend.loglike(Xo, Yo, eo, d, want_alpha=want_alpha, row_end=re)
             singles = [backend.loglike(Xo, Yo[:, c].contiguous(), eo, d, want_alpha=want_alpha, row_end=re)
                        for c in range(r)]
             assert int(info.item()) == 0
@@ -73,7 +73,7 @@ def test_multi_entries_against_single_output_runs(gpu_ready, case, r):
                 assert torch.equal(out, singles[0][0])
             assert float(out[0].item()) == pytest.approx(sum(ll), rel=1e-12)
             assert float(out[2].item()) == float(singles[0][0][2].item())    # logdet once, as the single output
-        g, _, galpha, _ = backend.loglike_grad_multi(Xo, Yo, eo, d, row_end=re)
+        g, _, galpha, _ = backend.loglike_grad(Xo, Yo, eo, d, row_end=re)
         gs = [backend.loglike_grad(Xo, Yo[:, c].contiguous(), eo, d, row_end=re)[0] for c in range(r)]
         k = len(gs[0])
         if r == 1:
@@ -82,8 +82,8 @@ def test_multi_entries_against_single_output_runs(gpu_ready, case, r):
         tot = torch.stack(gs).sum(dim=0)
         tot[2] = gs[0][2]                       # the joint record carries logdet once
         torch.testing.assert_close(g[:k], tot, rtol=1e-10, atol=1e-10 * float(tot[3:].abs().max()))
-        mt = backend.predict_mean_multi(Xs, Xo, d, alpha, truncate=True)
-        mf = backend.predict_mean_multi(Xs, Xo, d, alpha, truncate=False)
+        mt = backend.predict_mean(Xs, Xo, d, alpha, truncate=True)
+        mf = backend.predict_mean(Xs, Xo, d, alpha, truncate=False)
         for c in range(r):
             st = backend.predict_mean(Xs, Xo, d, alpha[:, c].contiguous(), truncate=True)
             assert torch.equal(mt[:, c], st), c
@@ -123,7 +123,7 @@ def test_multi_column_sweeps_equal_single_column_sweeps(gpu_ready, n):
             assert torch.equal(B[c, :n], singles[c]), (r, c)
 
 
-def test_full_multi_mean_equals_single_output_bit_for_bit(gpu_ready):
+def test_full_mean_of_columns_equals_single_output_bit_for_bit(gpu_ready):
     """With enough test points to fill the machine there is no split: each column of the full multi-output mean is its
     single-output mean bit for bit."""
     from treegp_b200 import backend
@@ -134,14 +134,14 @@ def test_full_multi_mean_equals_single_output_bit_for_bit(gpu_ready):
         Xd = backend.as_points(X)
         alpha = backend.to_device(Y)
         Xs = backend.as_points(np.random.default_rng(3).uniform(0, 300.0, size=(1 << 18, 2)))
-        m = backend.predict_mean_multi(Xs, Xd, d, alpha, truncate=False)
+        m = backend.predict_mean(Xs, Xd, d, alpha, truncate=False)
         for c in range(3):
             assert torch.equal(m[:, c], backend.predict_mean(Xs, Xd, d, alpha[:, c].contiguous(), truncate=False))
 
 
 @pytest.mark.parametrize("banded", [False, True])
 @pytest.mark.parametrize("case", list(CASES))
-def test_joint_loglike_and_gradient_against_the_oracle(gpu_ready, monkeypatch, case, banded):
+def test_joint_loglike_and_gradient_of_columns_against_the_oracle(gpu_ready, monkeypatch, case, banded):
     from treegp_b200 import backend
     from treegp_b200.kernels import lower_jacobian
     from treegp_b200.log_likelihood import log_likelihood as LL
@@ -152,7 +152,7 @@ def test_joint_loglike_and_gradient_against_the_oracle(gpu_ready, monkeypatch, c
     Xo, Yo, eo, row_end = _sorted(X, d, Y, e2)
     if banded:
         assert row_end[0] < 700
-    out = backend.loglike_grad_multi(Xo, Yo, eo, d, row_end=row_end if banded else None)[0].cpu().numpy()
+    out = backend.loglike_grad(Xo, Yo, eo, d, row_end=row_end if banded else None)[0].cpu().numpy()
     terms, white = so.terms_of(backend.as_sum(d))
     ll, g, _ = mo.joint_log_likelihood_gradient(terms, white, X, Y, e2)
     assert out[0] == pytest.approx(ll, rel=1e-10)
@@ -175,7 +175,7 @@ def test_joint_loglike_and_gradient_against_the_oracle(gpu_ready, monkeypatch, c
     np.testing.assert_allclose(gt, fd, rtol=2e-5, atol=1e-6 * np.max(np.abs(gt)))
 
 
-def test_repeated_calls_are_bit_identical_and_failures_give_minus_inf(gpu_ready):
+def test_repeated_calls_with_columns_are_bit_identical_and_failures_give_minus_inf(gpu_ready):
     from treegp_b200 import backend
 
     d = _desc(CASES["sum_white"])
@@ -183,17 +183,17 @@ def test_repeated_calls_are_bit_identical_and_failures_give_minus_inf(gpu_ready)
     Xo, Yo, eo, row_end = _sorted(X, d, Y, e2)
     Xs = backend.as_points(np.random.default_rng(1).uniform(0, 300.0, size=(30000, 2)))
     for re in (None, row_end):
-        a = backend.loglike_grad_multi(Xo, Yo, eo, d, row_end=re)
-        b = backend.loglike_grad_multi(Xo, Yo, eo, d, row_end=re)
+        a = backend.loglike_grad(Xo, Yo, eo, d, row_end=re)
+        b = backend.loglike_grad(Xo, Yo, eo, d, row_end=re)
         assert torch.equal(a[0], b[0]) and torch.equal(a[2], b[2])
-        assert torch.equal(backend.predict_mean_multi(Xs, Xo, d, a[2], truncate=True),
-                           backend.predict_mean_multi(Xs, Xo, d, a[2], truncate=True))
+        assert torch.equal(backend.predict_mean(Xs, Xo, d, a[2], truncate=True),
+                           backend.predict_mean(Xs, Xo, d, a[2], truncate=True))
         bad = eo.clone()
         bad[100] = -1e3                         # not positive definite
-        out, info, _, _ = backend.loglike_grad_multi(Xo, Yo, bad, d, row_end=re)
+        out, info, _, _ = backend.loglike_grad(Xo, Yo, bad, d, row_end=re)
         o = out.cpu().numpy()
         assert int(info.item()) > 0 and o[0] == -np.inf and np.all(o[3:] == 0.0)
-        assert float(backend.loglike_multi(Xo, Yo, bad, d, row_end=re)[0][0].item()) == -np.inf
+        assert float(backend.loglike(Xo, Yo, bad, d, row_end=re)[0][0].item()) == -np.inf
 
 
 @pytest.mark.parametrize("banded", [False, True])

@@ -4,7 +4,7 @@
     envelope factorisation): tgp_loglike_multi and tgp_loglike_grad_multi for r = 2 and 8 outputs against r
     single-output calls on the same data; and both triangular sweeps on the N = 40k factor for r = 1, 2, 4, 8 columns
     in one pass (tgp_potrs_multi) against r single-column solves (tgp_potrs_vec).  CUDA events, the arms alternated, five rounds after a warm-up of each.
-  * the truncated mean at M = 1e6 test points for r = 2 and 8 (backend.predict_mean_multi) against r calls of
+  * the truncated mean at M = 1e6 test points for r = 2 and 8 (backend.predict_mean with alpha (N, r)) against r calls of
     backend.predict_mean (Hilbert sort included in both).
   * configs[1] size (N = 10k, c * AnisotropicRBF): the public fit ("log-likelihood", analytic gradient) plus predict at
     1e5 points of a 2-output field, against two single-output GPInterpolations; wall time, alternated twice after a
@@ -78,13 +78,13 @@ def cfg2(treegp, backend):
         Yr = Yo[:, :r].contiguous()
         cols = [Yr[:, c].contiguous() for c in range(r)]
         rec["loglike_env_r%d_ms" % r] = alternate({
-            "multi": lambda: backend.loglike_multi(Xo, Yr, eo, d, work=work, row_end=row_end),
+            "multi": lambda: backend.loglike(Xo, Yr, eo, d, work=work, row_end=row_end),
             "singles": lambda: [backend.loglike(Xo, y, eo, d, work=work, row_end=row_end) for y in cols]})
         rec["loglike_grad_env_r%d_ms" % r] = alternate({
-            "multi": lambda: backend.loglike_grad_multi(Xo, Yr, eo, d, work=work, row_end=row_end),
+            "multi": lambda: backend.loglike_grad(Xo, Yr, eo, d, work=work, row_end=row_end),
             "singles": lambda: [backend.loglike_grad(Xo, y, eo, d, work=work, row_end=row_end) for y in cols]},
             rounds=3)
-        m = backend.loglike_multi(Xo, Yr, eo, d, work=work, row_end=row_end)[0].cpu().numpy()
+        m = backend.loglike(Xo, Yr, eo, d, work=work, row_end=row_end)[0].cpu().numpy()
         s = [float(backend.loglike(Xo, y, eo, d, work=work, row_end=row_end)[0][0].item()) for y in cols]
         rec["joint_logL_r%d" % r] = float(m[0])
         rec["sum_single_logL_r%d" % r] = float(sum(s))
@@ -107,7 +107,7 @@ def cfg2(treegp, backend):
         acols = [ar[:, c].contiguous() for c in range(r)]
         res = {}
         rec["predict_mean_trunc_M1e6_r%d_ms" % r] = alternate({
-            "multi": lambda: res.__setitem__("m", backend.predict_mean_multi(Xs, Xo, d, ar, truncate=True)),
+            "multi": lambda: res.__setitem__("m", backend.predict_mean(Xs, Xo, d, ar, truncate=True)),
             "singles": lambda: res.__setitem__("s", [backend.predict_mean(Xs, Xo, d, a, truncate=True)
                                                      for a in acols])}, rounds=3)
         rec["predict_mean_trunc_r%d_columns_bit_identical" % r] = bool(all(

@@ -71,6 +71,31 @@ def is_sum(kdesc):
     return isinstance(kdesc, TgpKernelSum)
 
 
+def as_sum(kdesc):
+    """The descriptor as a TgpKernelSum (the *_sum and multi-output entries): a TgpKernel becomes a one-term sum
+    without white, which those entries hand to the single-term entries, bit for bit."""
+    if is_sum(kdesc):
+        return kdesc
+    s = TgpKernelSum()
+    s.nterms, s.ndim, s.white = 1, kdesc.ndim, 0.0
+    s.term[0] = kdesc
+    return s
+
+
+def _outputs(v, N, name):
+    """Number of outputs r of `v`: (N,) is one output, (N, r) r of them with 1 <= r <= MAX_RHS."""
+    r = 1 if v.dim() == 1 else int(v.shape[1]) if v.dim() == 2 else 0
+    if not (1 <= r <= _cabi.MAX_RHS and v.shape[0] == N):
+        raise ValueError("%s must have shape (N,) or (N, r) = (%d, r) with 1 <= r <= %d; got %r"
+                         % (name, N, _cabi.MAX_RHS, tuple(v.shape)))
+    return r
+
+
+def _envelope(row_end):
+    """(pointer, block count) of an optional envelope (envelope_rows) for the C entries."""
+    return (None, 0) if row_end is None else (_host_i64(row_end), len(row_end))
+
+
 def kmat_sym(X, kdesc, diag_add=None, out=None, lower_only=False):
     """K(X,X) + diag(diag_add).  Returns the (N, ld) workspace; the matrix is out[:, :N].  kdesc: TgpKernel or
     TgpKernelSum (every function here that takes a descriptor accepts both)."""
@@ -79,10 +104,8 @@ def kmat_sym(X, kdesc, diag_add=None, out=None, lower_only=False):
     N = X.shape[0]
     if out is None:
         out = alloc_matrix(N, N, X.device)
-    lib = _cabi.load()
-    fn = lib.tgp_kmat_sym_sum if is_sum(kdesc) else lib.tgp_kmat_sym
-    check(fn(_p(X), N, ctypes.byref(kdesc), _p(diag_add), _p(out), out.stride(0), int(bool(lower_only)), _stream()),
-          fn.__name__)
+    check(_cabi.load().tgp_kmat_sym_sum(_p(X), N, ctypes.byref(as_sum(kdesc)), _p(diag_add), _p(out), out.stride(0),
+                                        int(bool(lower_only)), _stream()), "tgp_kmat_sym_sum")
     return out
 
 
@@ -92,9 +115,8 @@ def kmat_cross(Xs, X, kdesc, out=None):
     M, N = Xs.shape[0], X.shape[0]
     if out is None:
         out = alloc_matrix(M, N, X.device)
-    lib = _cabi.load()
-    fn = lib.tgp_kmat_cross_sum if is_sum(kdesc) else lib.tgp_kmat_cross
-    check(fn(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(out), out.stride(0), _stream()), fn.__name__)
+    check(_cabi.load().tgp_kmat_cross_sum(_p(Xs), M, _p(X), N, ctypes.byref(as_sum(kdesc)), _p(out), out.stride(0),
+                                          _stream()), "tgp_kmat_cross_sum")
     return out
 
 
@@ -217,31 +239,35 @@ def logdet_chi2(L, N, y=None, alpha=None):
     return out
 
 
-def loglike(X, y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
-    """One marginal-likelihood evaluation.  Returns (out[3] = logL, chi2, logdet; info; alpha; work).
-    row_end: X (with y, yerr2) is sorted along an axis and the factorisation stays inside that envelope
-    (plan_envelope; tgp_loglike_env)."""
+def _solve_args(X, y, yerr2, work, name):
+    """Points, N, the number of outputs r of y ((N,) or (N, r)) and a workspace of N + r rows (the outputs ride
+    through the factorisation as extra rows)."""
     X = as_points(X)
     N = X.shape[0]
+    r = _outputs(y, N, "y")
+    if yerr2 is not None and tuple(yerr2.shape) != (N,):
+        raise ValueError("yerr2 must have shape (N,) = (%d,); got %r" % (N, tuple(yerr2.shape)))
     if work is None:
-        work = alloc_matrix(N + 1, N, X.device)
-    if work.shape[0] < N + 1:
-        raise ValueError("loglike workspace needs N+1 rows")
-    alpha = torch.empty(N, dtype=F64, device=X.device)
+        work = alloc_matrix(N + r, N, X.device)
+    if work.shape[0] < N + r:
+        raise ValueError("%s workspace needs N+%d rows" % (name, r))
+    return X, N, r, work
+
+
+def loglike(X, y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
+    """One marginal-likelihood evaluation (tgp_loglike_multi).  y: (N,), or (N, r) for r outputs sharing the kernel,
+    whose joint logL is the sum of theirs.  Returns (out[3] = logL, chi2, logdet; info; alpha, shaped as y; work,
+    N + r rows).  row_end: X (with y, yerr2) is sorted along an axis and the factorisation stays inside that envelope
+    (plan_envelope)."""
+    X, N, r, work = _solve_args(X, y, yerr2, work, "loglike")
+    y = y.contiguous()
+    alpha = torch.empty(y.shape, dtype=F64, device=X.device)
     out = torch.zeros(3, dtype=F64, device=X.device)
     info = torch.zeros(1, dtype=torch.int32, device=X.device)
-    if is_sum(kdesc):
-        re = None if row_end is None else _host_i64(row_end)
-        check(_cabi.load().tgp_loglike_sum(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
-                                           _p(alpha), int(bool(want_alpha)), _p(out), _p(info), re,
-                                           0 if row_end is None else len(row_end), _stream()), "tgp_loglike_sum")
-    elif row_end is None:
-        check(_cabi.load().tgp_loglike(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
-                                       _p(alpha), int(bool(want_alpha)), _p(out), _p(info), _stream()), "tgp_loglike")
-    else:
-        check(_cabi.load().tgp_loglike_env(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
-                                           _p(alpha), int(bool(want_alpha)), _p(out), _p(info), _host_i64(row_end),
-                                           len(row_end), _stream()), "tgp_loglike_env")
+    re, nre = _envelope(row_end)
+    check(_cabi.load().tgp_loglike_multi(_p(X), _p(y), r, _p(yerr2), N, ctypes.byref(as_sum(kdesc)), _p(work),
+                                         work.stride(0), _p(alpha), int(bool(want_alpha)), _p(out), _p(info), re, nre,
+                                         _stream()), "tgp_loglike_multi")
     return out, info, alpha, work
 
 
@@ -271,94 +297,33 @@ def selinv_flops(row_end, n):
 
 
 def loglike_grad(X, y, yerr2, kdesc, work=None, row_end=None):
-    """Log-likelihood and its gradient in one call (tgp_loglike_grad).  Returns (out[7] = logL, chi2, logdet,
-    d logL / d ln amp, d logL / d m00, d m01, d m11; info; alpha = K^-1 y; work, which holds Z = K^-1 inside the
-    envelope afterwards).  row_end as for loglike (X, y, yerr2 sorted along the envelope's axis).  For a sum
-    (tgp_loglike_grad_sum) out has 4 + 4 nterms entries: the four derivatives per term, then d logL / d ln white."""
-    X = as_points(X)
+    """Log-likelihood and its gradient in one call.  Returns (out; info; alpha = K^-1 y, shaped as y; work, which holds
+    Z = K^-1 inside the envelope afterwards).  y and row_end as for loglike.  A TgpKernel with y of shape (N,)
+    (tgp_loglike_grad): out[7] = logL, chi2, logdet, d logL / d ln amp, d logL / d m00, d m01, d m11.  A sum, or r
+    outputs (tgp_loglike_grad_multi: the joint logL): out has 4 + 4 nterms entries, the four derivatives per term,
+    then d logL / d ln white; a TgpKernel counts as one term."""
+    X, N, r, work = _solve_args(X, y, yerr2, work, "loglike_grad")
     _check_dims(kdesc, X)
-    N = X.shape[0]
-    if work is None:
-        work = alloc_matrix(N + 1, N, X.device)
-    if work.shape[0] < N + 1:
-        raise ValueError("loglike_grad workspace needs N+1 rows")
-    alpha = torch.empty(N, dtype=F64, device=X.device)
+    y = y.contiguous()
+    alpha = torch.empty(y.shape, dtype=F64, device=X.device)
     info = torch.zeros(1, dtype=torch.int32, device=X.device)
+    re, nre = _envelope(row_end)
     lib = _cabi.load()
-    if is_sum(kdesc):
-        out = torch.zeros(4 + 4 * kdesc.nterms, dtype=F64, device=X.device)
-        scratch = torch.empty(int(lib.tgp_loglike_grad_sum_work_doubles(int(N), int(kdesc.nterms))), dtype=F64,
-                              device=X.device)
-        fn = lib.tgp_loglike_grad_sum
-    else:
+    if y.dim() == 1 and not is_sum(kdesc):
+        # the single-term entry: as a one-term sum it would take one more launch (clearing d / d ln white) and a
+        # larger scratch
         out = torch.zeros(7, dtype=F64, device=X.device)
-        scratch = _selinv_scratch(N, X.device)
-        fn = lib.tgp_loglike_grad
-    re = None if row_end is None else _host_i64(row_end)
-    check(fn(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0), _p(alpha), _p(out), _p(info),
-             re, 0 if row_end is None else len(row_end), _p(scratch), _stream()), fn.__name__)
-    return out, info, alpha, work
-
-
-def as_sum(kdesc):
-    """The descriptor as a TgpKernelSum (the multi-output entries take sums only): a TgpKernel becomes a one-term sum
-    without white, which the device runs with the single-term kernels."""
-    if is_sum(kdesc):
-        return kdesc
-    s = TgpKernelSum()
-    s.nterms, s.ndim, s.white = 1, kdesc.ndim, 0.0
-    s.term[0] = kdesc
-    return s
-
-
-def _multi_args(X, Y, yerr2, work, rows_needed):
-    X = as_points(X)
-    N = X.shape[0]
-    if Y.dim() != 2 or Y.shape[0] != N or not 1 <= Y.shape[1] <= _cabi.MAX_RHS:
-        raise ValueError("Y must have shape (N, r) with 1 <= r <= %d; got %r" % (_cabi.MAX_RHS, tuple(Y.shape)))
-    if yerr2 is not None and tuple(yerr2.shape) != (N,):
-        raise ValueError("yerr2 must have shape (N,) = (%d,); got %r" % (N, tuple(yerr2.shape)))
-    r = int(Y.shape[1])
-    if work is None:
-        work = alloc_matrix(N + r, N, X.device)
-    if work.shape[0] < N + r:
-        raise ValueError("%s workspace needs N+r rows" % rows_needed)
-    return X, N, r, work
-
-
-def loglike_multi(X, Y, yerr2, kdesc, work=None, want_alpha=False, row_end=None):
-    """loglike for r outputs sharing the kernel (tgp_loglike_multi): Y (N, r) device tensor.  Returns (out[3] =
-    joint logL, sum of chi2, logdet; info; alpha (N, r); work, N + r rows)."""
-    X, N, r, work = _multi_args(X, Y, yerr2, work, "loglike_multi")
-    Y = Y.contiguous()
-    alpha = torch.empty((N, r), dtype=F64, device=X.device)
-    out = torch.zeros(3, dtype=F64, device=X.device)
-    info = torch.zeros(1, dtype=torch.int32, device=X.device)
-    re = None if row_end is None else _host_i64(row_end)
-    check(_cabi.load().tgp_loglike_multi(_p(X), _p(Y), r, _p(yerr2), N, ctypes.byref(as_sum(kdesc)), _p(work),
-                                         work.stride(0), _p(alpha), int(bool(want_alpha)), _p(out), _p(info), re,
-                                         0 if row_end is None else len(row_end), _stream()), "tgp_loglike_multi")
-    return out, info, alpha, work
-
-
-def loglike_grad_multi(X, Y, yerr2, kdesc, work=None, row_end=None):
-    """loglike_grad for r outputs (tgp_loglike_grad_multi): the joint logL and its gradient, out in the layout of
-    tgp_loglike_grad_sum (4 + 4 nterms entries; a TgpKernel counts as one term).  Returns (out, info, alpha (N, r),
-    work)."""
-    X, N, r, work = _multi_args(X, Y, yerr2, work, "loglike_grad_multi")
-    _check_dims(kdesc, X)
-    Y = Y.contiguous()
+        check(lib.tgp_loglike_grad(_p(X), _p(y), _p(yerr2), N, ctypes.byref(kdesc), _p(work), work.stride(0),
+                                   _p(alpha), _p(out), _p(info), re, nre, _p(_selinv_scratch(N, X.device)), _stream()),
+              "tgp_loglike_grad")
+        return out, info, alpha, work
     ks = as_sum(kdesc)
-    lib = _cabi.load()
-    alpha = torch.empty((N, r), dtype=F64, device=X.device)
-    info = torch.zeros(1, dtype=torch.int32, device=X.device)
     out = torch.zeros(4 + 4 * ks.nterms, dtype=F64, device=X.device)
     scratch = torch.empty(int(lib.tgp_loglike_grad_multi_work_doubles(int(N), int(ks.nterms), r)), dtype=F64,
                           device=X.device)
-    re = None if row_end is None else _host_i64(row_end)
-    check(lib.tgp_loglike_grad_multi(_p(X), _p(Y), r, _p(yerr2), N, ctypes.byref(ks), _p(work), work.stride(0),
-                                     _p(alpha), _p(out), _p(info), re, 0 if row_end is None else len(row_end),
-                                     _p(scratch), _stream()), "tgp_loglike_grad_multi")
+    check(lib.tgp_loglike_grad_multi(_p(X), _p(y), r, _p(yerr2), N, ctypes.byref(ks), _p(work), work.stride(0),
+                                     _p(alpha), _p(out), _p(info), re, nre, _p(scratch), _stream()),
+          "tgp_loglike_grad_multi")
     return out, info, alpha, work
 
 
@@ -493,54 +458,28 @@ TRUNC_MIN_M, TRUNC_MIN_N = 16384, 2048   # below this the plain kernel is launch
 
 
 def predict_mean(Xs, X, kdesc, alpha, out=None, truncate=None):
-    """mean = K(Xs, X) . alpha without materialising K(Xs, X) (gp_interp.py:177,183).
+    """mean = K(Xs, X) . alpha without materialising K(Xs, X) (gp_interp.py:177,183); alpha (N,) gives mean (M,),
+    alpha (N, r) of r outputs mean (M, r), every pair's profile evaluated once for all outputs
+    (tgp_predict_mean[_trunc]_multi).
 
     truncate=True (default for large problems): both point sets are put in Hilbert-curve order (torch argsort /
-    gather: plumbing) and tgp_predict_mean_trunc skips blocks of pairs whose correlation is provably below
+    gather: plumbing) and the truncated entry skips blocks of pairs whose correlation is provably below
     1e-40; the result differs from the full sum by at most 1e-40 * sum|amp alpha| (and by summation order)."""
     Xs, X = as_points(Xs), as_points(X)
     _check_dims(kdesc, X, Xs)
     M, N = Xs.shape[0], X.shape[0]
+    r = _outputs(alpha, N, "alpha")
+    alpha = alpha.contiguous()
+    shape = (M,) + tuple(alpha.shape[1:])
     if out is None:
-        out = torch.empty(M, dtype=F64, device=X.device)
-    lib = _cabi.load()
-    if truncate is None:
-        truncate = M >= TRUNC_MIN_M and N >= TRUNC_MIN_N
-    if not truncate:
-        fn = lib.tgp_predict_mean_sum if is_sum(kdesc) else lib.tgp_predict_mean
-        check(fn(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(alpha), _p(out), _stream()), fn.__name__)
-        return out
-    two_d = X.shape[1] == 2
-    zt, zs = torch.zeros(N, dtype=F64, device=X.device), torch.zeros(M, dtype=F64, device=X.device)
-    ot = hilbert_order(X[:, 0].contiguous(), X[:, 1].contiguous() if two_d else zt)
-    os_ = hilbert_order(Xs[:, 0].contiguous(), Xs[:, 1].contiguous() if two_d else zs)
-    Xt, at, Xss = X[ot].contiguous(), alpha[ot].contiguous(), Xs[os_].contiguous()
-    work = torch.empty(int(lib.tgp_predict_work_doubles(N)), dtype=F64, device=X.device)
-    tmp = torch.empty(M, dtype=F64, device=X.device)
-    fn = lib.tgp_predict_mean_trunc_sum if is_sum(kdesc) else lib.tgp_predict_mean_trunc
-    check(fn(_p(Xss), M, _p(Xt), N, ctypes.byref(kdesc), _p(at), _p(tmp), _p(work), _stream()), fn.__name__)
-    out[os_] = tmp
-    return out
-
-
-def predict_mean_multi(Xs, X, kdesc, alpha, truncate=None):
-    """predict_mean for r outputs (tgp_predict_mean[_trunc]_multi): alpha (N, r) -> mean (M, r); every pair's
-    profile is evaluated once for all outputs.  Same Hilbert ordering and truncation choice as predict_mean."""
-    Xs, X = as_points(Xs), as_points(X)
-    _check_dims(kdesc, X, Xs)
-    M, N = Xs.shape[0], X.shape[0]
-    if alpha.dim() != 2 or alpha.shape[0] != N or not 1 <= alpha.shape[1] <= _cabi.MAX_RHS:
-        raise ValueError("alpha must have shape (N, r) = (%d, r) with 1 <= r <= %d; got %r"
-                         % (N, _cabi.MAX_RHS, tuple(alpha.shape)))
-    r = int(alpha.shape[1])
+        out = torch.empty(shape, dtype=F64, device=X.device)
     ks = as_sum(kdesc)
     lib = _cabi.load()
     if truncate is None:
         truncate = M >= TRUNC_MIN_M and N >= TRUNC_MIN_N
-    out = torch.empty((M, r), dtype=F64, device=X.device)
     if not truncate:
-        check(lib.tgp_predict_mean_multi(_p(Xs), M, _p(X), N, ctypes.byref(ks), _p(alpha.contiguous()), r, _p(out),
-                                         _stream()), "tgp_predict_mean_multi")
+        check(lib.tgp_predict_mean_multi(_p(Xs), M, _p(X), N, ctypes.byref(ks), _p(alpha), r, _p(out), _stream()),
+              "tgp_predict_mean_multi")
         return out
     two_d = X.shape[1] == 2
     zt, zs = torch.zeros(N, dtype=F64, device=X.device), torch.zeros(M, dtype=F64, device=X.device)
@@ -548,7 +487,7 @@ def predict_mean_multi(Xs, X, kdesc, alpha, truncate=None):
     os_ = hilbert_order(Xs[:, 0].contiguous(), Xs[:, 1].contiguous() if two_d else zs)
     Xt, at, Xss = X[ot].contiguous(), alpha[ot].contiguous(), Xs[os_].contiguous()
     work = torch.empty(int(lib.tgp_predict_work_doubles(N)), dtype=F64, device=X.device)
-    tmp = torch.empty((M, r), dtype=F64, device=X.device)
+    tmp = torch.empty(shape, dtype=F64, device=X.device)
     check(lib.tgp_predict_mean_trunc_multi(_p(Xss), M, _p(Xt), N, ctypes.byref(ks), _p(at), r, _p(tmp), _p(work),
                                            _stream()), "tgp_predict_mean_trunc_multi")
     out[os_] = tmp
@@ -577,9 +516,8 @@ def knn_mean(X0, y0, Xq, k):
 
 
 def predict_var(Xs, X, kdesc, L, chunk=None, out=None, work=None, row_end=None):
-    """Diagonal predictive variance amp - |L^-1 k*|^2 (tgp_predict_var; a sum: sum_c amp_c + white - |L^-1 k*|^2,
-    tgp_predict_var_sum); row_end: the factor's envelope, X in the
-    factor's (sorted) order (tgp_predict_var_env)."""
+    """Diagonal predictive variance amp - |L^-1 k*|^2 (a sum: sum_c amp_c + white - |L^-1 k*|^2; tgp_predict_var_sum);
+    row_end: the factor's envelope, X in the factor's (sorted) order."""
     Xs, X = as_points(Xs), as_points(X)
     _check_dims(kdesc, X, Xs)
     M, N = Xs.shape[0], X.shape[0]
@@ -591,18 +529,9 @@ def predict_var(Xs, X, kdesc, L, chunk=None, out=None, work=None, row_end=None):
         work = torch.empty(chunk * (N + 1), dtype=F64, device=X.device)
     if out is None:
         out = torch.empty(M, dtype=F64, device=X.device)
-    if is_sum(kdesc):
-        check(_cabi.load().tgp_predict_var_sum(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(L), L.stride(0),
-                                               None if row_end is None else _host_i64(row_end),
-                                               0 if row_end is None else len(row_end), _p(work), chunk, _p(out),
-                                               _stream()), "tgp_predict_var_sum")
-    elif row_end is None:
-        check(_cabi.load().tgp_predict_var(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(L), L.stride(0), _p(work),
-                                           chunk, _p(out), _stream()), "tgp_predict_var")
-    else:
-        check(_cabi.load().tgp_predict_var_env(_p(Xs), M, _p(X), N, ctypes.byref(kdesc), _p(L), L.stride(0),
-                                               _host_i64(row_end), len(row_end), _p(work), chunk, _p(out), _stream()),
-              "tgp_predict_var_env")
+    re, nre = _envelope(row_end)
+    check(_cabi.load().tgp_predict_var_sum(_p(Xs), M, _p(X), N, ctypes.byref(as_sum(kdesc)), _p(L), L.stride(0), re,
+                                           nre, _p(work), chunk, _p(out), _stream()), "tgp_predict_var_sum")
     return out
 
 

@@ -1144,12 +1144,15 @@ static int loglike_after_build(const double* y, int64_t N, double* work, int64_t
   return TGP_OK;
 }
 
+// k or ks (the other NULL): single-term or sum kernel
 static int loglike_impl(const double* X, const double* y, const double* yerr2, int64_t N,
-                        const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
-                        double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
+                        const tgp_kernel* k, const tgp_kernel_sum* ks, double* work, int64_t ld, double* alpha,
+                        int want_alpha, double* out, int32_t* info, const int64_t* row_end, int64_t nblocks,
+                        void* stream) {
   int rc = loglike_args(X, y, N, work, alpha, out, info, row_end, nblocks);
   if (rc) return rc;
-  rc = tgp_kmat_sym(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
+  rc = ks ? tgp_kmat_sym_sum(X, N, ks, yerr2, work, ld, /*lower_only=*/1, stream)
+          : tgp_kmat_sym(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
   if (rc) return rc;
   return loglike_after_build(y, N, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
 }
@@ -1157,24 +1160,20 @@ static int loglike_impl(const double* X, const double* y, const double* yerr2, i
 extern "C" int tgp_loglike(const double* X, const double* y, const double* yerr2, int64_t N,
                            const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
                            double* out, int32_t* info, void* stream) {
-  return loglike_impl(X, y, yerr2, N, k, work, ld, alpha, want_alpha, out, info, nullptr, 0, stream);
+  return loglike_impl(X, y, yerr2, N, k, nullptr, work, ld, alpha, want_alpha, out, info, nullptr, 0, stream);
 }
 
 extern "C" int tgp_loglike_env(const double* X, const double* y, const double* yerr2, int64_t N,
                                const tgp_kernel* k, double* work, int64_t ld, double* alpha, int want_alpha,
                                double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
   TGP_CHECK_ARG(row_end != nullptr, "row_end");
-  return loglike_impl(X, y, yerr2, N, k, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+  return loglike_impl(X, y, yerr2, N, k, nullptr, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
 }
 
 extern "C" int tgp_loglike_sum(const double* X, const double* y, const double* yerr2, int64_t N,
                                const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, int want_alpha,
                                double* out, int32_t* info, const int64_t* row_end, int64_t nblocks, void* stream) {
-  int rc = loglike_args(X, y, N, work, alpha, out, info, row_end, nblocks);
-  if (rc) return rc;
-  rc = tgp_kmat_sym_sum(X, N, k, yerr2, work, ld, /*lower_only=*/1, stream);
-  if (rc) return rc;
-  return loglike_after_build(y, N, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
+  return loglike_impl(X, y, yerr2, N, nullptr, k, work, ld, alpha, want_alpha, out, info, row_end, nblocks, stream);
 }
 
 // ============================================================================================

@@ -201,40 +201,52 @@ kmat_cross_kernel(const double* __restrict__ Xs, int64_t M, const double* __rest
 }
 
 // ---- C ABI -----------------------------------------------------------------------------------
-extern "C" int tgp_kmat_sym(const double* X, int64_t N, const tgp_kernel* k, const double* diag_add,
-                            double* out, int64_t ld, int lower_only, void* stream) {
-  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+// The checks, geometry and launch of one build; the entries below only validate the descriptor and pick the profile.
+template <class P>
+static int kmat_sym_launch(const double* X, int64_t N, const P& prof, const double* diag_add, double* out, int64_t ld,
+                           int lower_only, void* stream) {
   TGP_CHECK_ARG(N >= 0 && ld >= N, "N/ld");
   if (N == 0) return TGP_OK;
   TGP_CHECK_ARG(X && out, "null pointer");
-  const KDesc kd = make_kdesc(k);
   const int64_t nt = tgp_cdiv(N, KT);
   const int64_t ntiles = nt * (nt + 1) / 2;
   TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
   const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
-  cudaStream_t st = (cudaStream_t)stream;
-  const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (kmat_sym_kernel<FamilyProfile<FAM>><<<(unsigned)ntiles, KT_THREADS, 0, st>>>(
-                                   X, N, FamilyProfile<FAM>{kd}, diag_add, out, ld, lower_only, vec_ok, phi)));
+  kmat_sym_kernel<P><<<(unsigned)ntiles, KT_THREADS, 0, (cudaStream_t)stream>>>(X, N, prof, diag_add, out, ld,
+                                                                               lower_only, vec_ok, tgp_phi_device());
   TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+template <class P>
+static int kmat_cross_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof, double* out,
+                             int64_t ld, void* stream) {
+  TGP_CHECK_ARG(M >= 0 && N >= 0 && ld >= N, "M/N/ld");
+  if (M == 0 || N == 0) return TGP_OK;
+  TGP_CHECK_ARG(Xs && X && out, "null pointer");
+  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
+  dim3 grid((unsigned)tgp_cdiv(M, KT), (unsigned)tgp_cdiv(N, KT));  // x: row tiles (M may be millions)
+  TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
+  kmat_cross_kernel<P><<<grid, KT_THREADS, 0, (cudaStream_t)stream>>>(Xs, M, X, N, prof, out, ld, vec_ok,
+                                                                      tgp_phi_device());
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+extern "C" int tgp_kmat_sym(const double* X, int64_t N, const tgp_kernel* k, const double* diag_add,
+                            double* out, int64_t ld, int lower_only, void* stream) {
+  TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
+  const KDesc kd = make_kdesc(k);
+  TGP_FAMILY_SWITCH(k->family, return kmat_sym_launch(X, N, FamilyProfile<FAM>{kd}, diag_add, out, ld, lower_only,
+                                                      stream));
   return TGP_OK;
 }
 
 extern "C" int tgp_kmat_cross(const double* Xs, int64_t M, const double* X, int64_t N,
                               const tgp_kernel* k, double* out, int64_t ld, void* stream) {
   TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
-  TGP_CHECK_ARG(M >= 0 && N >= 0 && ld >= N, "M/N/ld");
-  if (M == 0 || N == 0) return TGP_OK;
-  TGP_CHECK_ARG(Xs && X && out, "null pointer");
   const KDesc kd = make_kdesc(k);
-  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
-  dim3 grid((unsigned)tgp_cdiv(M, KT), (unsigned)tgp_cdiv(N, KT));  // x: row tiles (M may be millions)
-  TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
-  cudaStream_t st = (cudaStream_t)stream;
-  const double* phi = tgp_phi_device();
-  TGP_FAMILY_SWITCH(k->family, (kmat_cross_kernel<FamilyProfile<FAM>><<<grid, KT_THREADS, 0, st>>>(
-                                   Xs, M, X, N, FamilyProfile<FAM>{kd}, out, ld, vec_ok, phi)));
-  TGP_LAUNCH_CHECK();
+  TGP_FAMILY_SWITCH(k->family, return kmat_cross_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, out, ld, stream));
   return TGP_OK;
 }
 
@@ -243,33 +255,14 @@ extern "C" int tgp_kmat_sym_sum(const double* X, int64_t N, const tgp_kernel_sum
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   if (k->nterms == 1 && k->white == 0.0)   // one term: the single-term kernel, bit for bit
     return tgp_kmat_sym(X, N, &k->term[0], diag_add, out, ld, lower_only, stream);
-  TGP_CHECK_ARG(N >= 0 && ld >= N, "N/ld");
-  if (N == 0) return TGP_OK;
-  TGP_CHECK_ARG(X && out, "null pointer");
-  const int64_t nt = tgp_cdiv(N, KT);
-  const int64_t ntiles = nt * (nt + 1) / 2;
-  TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
-  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
-  kmat_sym_kernel<SumProfile><<<(unsigned)ntiles, KT_THREADS, 0, (cudaStream_t)stream>>>(
-      X, N, SumProfile{make_ksumdesc(k)}, diag_add, out, ld, lower_only, vec_ok, tgp_phi_device());
-  TGP_LAUNCH_CHECK();
-  return TGP_OK;
+  return kmat_sym_launch(X, N, SumProfile{make_ksumdesc(k)}, diag_add, out, ld, lower_only, stream);
 }
 
 extern "C" int tgp_kmat_cross_sum(const double* Xs, int64_t M, const double* X, int64_t N,
                                   const tgp_kernel_sum* k, double* out, int64_t ld, void* stream) {
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   if (k->nterms == 1) return tgp_kmat_cross(Xs, M, X, N, &k->term[0], out, ld, stream);   // no white in K(Xs, X)
-  TGP_CHECK_ARG(M >= 0 && N >= 0 && ld >= N, "M/N/ld");
-  if (M == 0 || N == 0) return TGP_OK;
-  TGP_CHECK_ARG(Xs && X && out, "null pointer");
-  const int vec_ok = (ld % 2 == 0) && (((uintptr_t)out & 15) == 0);
-  dim3 grid((unsigned)tgp_cdiv(M, KT), (unsigned)tgp_cdiv(N, KT));
-  TGP_CHECK_ARG(grid.y <= 65535u, "N too large for one launch");
-  kmat_cross_kernel<SumProfile><<<grid, KT_THREADS, 0, (cudaStream_t)stream>>>(
-      Xs, M, X, N, SumProfile{make_ksumdesc(k)}, out, ld, vec_ok, tgp_phi_device());
-  TGP_LAUNCH_CHECK();
-  return TGP_OK;
+  return kmat_cross_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, out, ld, stream);
 }
 
 // ---- batches of independent problems (tgp_loglike_batch) ---------------------------------------------------------

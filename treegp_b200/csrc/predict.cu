@@ -110,25 +110,46 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
   }
 }
 
+// columns of alpha and mean
 template <class P>
-static int predict_mean_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof,
-                               const double* alpha, double* mean, void* stream) {
+static int64_t mean_outputs(const P& prof) {
+  if constexpr (OutputsOf<P>::kR > 1) return prof.nrhs;
+  return 1;
+}
+
+// The checks of every mean launch and its empty cases: nothing to do for M == 0, M x nout zero means for N == 0.
+// `done`: nothing is left to launch.
+static int predict_mean_args(const double* Xs, int64_t M, const double* X, int64_t N, const double* alpha,
+                             double* mean, int64_t nout, void* stream, bool& done) {
+  done = true;
   TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
   if (M == 0) return TGP_OK;
   TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha)), "null pointer");
+  if (N == 0) {
+    TGP_CUDA(cudaMemsetAsync(mean, 0, M * nout * sizeof(double), (cudaStream_t)stream));
+    return TGP_OK;
+  }
+  done = false;
+  return TGP_OK;
+}
+
+template <class P>
+static int predict_mean_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof,
+                               const double* alpha, double* mean, void* stream) {
+  const int64_t nout = mean_outputs(prof);
+  bool done;
+  const int rc = predict_mean_args(Xs, M, X, N, alpha, mean, nout, stream, done);
+  if (rc || done) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t gx = tgp_cdiv(M, PM_THREADS);
   constexpr int R = OutputsOf<P>::kR;
-  int64_t nout = 1;
-  if constexpr (R > 1) nout = prof.nrhs;
   const int64_t ntile = tgp_cdiv(N, (int64_t)(R == 1 ? PM_TILE : 2048 / R));
   int64_t nsplit = 1;
   const int64_t target = 4ll * tgp_num_sms();
   if (gx < target) nsplit = tgp_cdiv(target, gx);
   if (nsplit > ntile) nsplit = ntile > 0 ? ntile : 1;
   if (nsplit > 65535) nsplit = 65535;
-  if (nsplit > 1 || N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * nout * sizeof(double), st));
-  if (N == 0) return TGP_OK;
+  if (nsplit > 1) TGP_CUDA(cudaMemsetAsync(mean, 0, M * nout * sizeof(double), st));
   dim3 grid((unsigned)gx, (unsigned)nsplit);
   predict_mean_kernel<P><<<grid, PM_THREADS, 0, st>>>(Xs, M, X, N, prof, alpha, mean, tgp_phi_device());
   TGP_LAUNCH_CHECK();
@@ -335,10 +356,32 @@ static double metric_lmin(const tgp_kernel* k) {
   return lmin;
 }
 
-// r2cut: squared Euclidean distance beyond which every pair is below the cut-off (caller: > 0)
+// r2cut: squared Euclidean distance beyond which every pair is below the cut-off of each of the nterms terms.  A group
+// is skipped only when it is beyond the cut-off of every term: the union of the supports is the largest per-term
+// qcut_c / lmin(M_c).  Each skipped pair is below 1e-40 |amp_c| for every term, so the mean changes by at most
+// 1e-40 sum_c |amp_c| sum_n |alpha_n|.
+static int trunc_r2cut(const tgp_kernel* terms, int nterms, double& r2cut) {
+  r2cut = 0.0;
+  for (int c = 0; c < nterms; ++c) {
+    const double lmin = metric_lmin(&terms[c]);
+    TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
+    const double r2 = profile_qcut(terms[c].family) / lmin;
+    if (r2 > r2cut) r2cut = r2;
+  }
+  return TGP_OK;
+}
+
+// prof evaluates the nterms terms of `terms` (a single term, or a sum)
 template <class P>
 static int predict_mean_trunc_launch(const double* Xs, int64_t M, const double* X, int64_t N, const P& prof,
-                                     double r2cut, const double* alpha, double* mean, double* work, void* stream) {
+                                     const tgp_kernel* terms, int nterms, const double* alpha, double* mean,
+                                     double* work, void* stream) {
+  bool done;
+  int rc = predict_mean_args(Xs, M, X, N, alpha, mean, mean_outputs(prof), stream, done);
+  if (rc || done) return rc;
+  TGP_CHECK_ARG(work, "null pointer");
+  double r2cut;
+  if ((rc = trunc_r2cut(terms, nterms, r2cut))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t ngroups = tgp_cdiv(N, PG);
   point_boxes_kernel<<<(unsigned)tgp_cdiv(ngroups, 8), 256, 0, st>>>(X, N, prof.desc.ndim, work, ngroups);
@@ -352,111 +395,70 @@ static int predict_mean_trunc_launch(const double* Xs, int64_t M, const double* 
   return TGP_OK;
 }
 
-static int predict_mean_trunc_args(const double* Xs, int64_t M, const double* X, int64_t N, const double* alpha,
-                                   double* mean, double* work, void* stream) {
-  TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
-  if (M == 0) return TGP_OK;
-  TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha && work)), "null pointer");
-  if (N == 0) TGP_CUDA(cudaMemsetAsync(mean, 0, M * sizeof(double), (cudaStream_t)stream));
-  return TGP_OK;
-}
-
 extern "C" int tgp_predict_mean_trunc(const double* Xs, int64_t M, const double* X, int64_t N,
                                       const tgp_kernel* k, const double* alpha, double* mean, double* work,
                                       void* stream) {
   TGP_CHECK_ARG(kdesc_ok(k), "kernel descriptor");
-  const int rc = predict_mean_trunc_args(Xs, M, X, N, alpha, mean, work, stream);
-  if (rc || M == 0 || N == 0) return rc;
-  const double lmin = metric_lmin(k);
-  TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
-  const double r2cut = profile_qcut(k->family) / lmin;
   const KDesc kd = make_kdesc(k);
-  TGP_FAMILY_SWITCH(k->family, return predict_mean_trunc_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, r2cut, alpha,
+  TGP_FAMILY_SWITCH(k->family, return predict_mean_trunc_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, k, 1, alpha,
                                                                 mean, work, stream));
   return TGP_OK;
 }
 
-// A group is skipped only when it is beyond the cut-off of every term: the union of the supports is the largest
-// per-term qcut_c / lmin(M_c).  Each skipped pair is below 1e-40 |amp_c| for every term, so the mean changes by at
-// most 1e-40 sum_c |amp_c| sum_n |alpha_n|.
 extern "C" int tgp_predict_mean_trunc_sum(const double* Xs, int64_t M, const double* X, int64_t N,
                                           const tgp_kernel_sum* k, const double* alpha, double* mean, double* work,
                                           void* stream) {
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   if (k->nterms == 1) return tgp_predict_mean_trunc(Xs, M, X, N, &k->term[0], alpha, mean, work, stream);
-  const int rc = predict_mean_trunc_args(Xs, M, X, N, alpha, mean, work, stream);
-  if (rc || M == 0 || N == 0) return rc;
-  double r2cut = 0.0;
-  for (int c = 0; c < k->nterms; ++c) {
-    const double lmin = metric_lmin(&k->term[c]);
-    TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
-    const double r2 = profile_qcut(k->term[c].family) / lmin;
-    if (r2 > r2cut) r2cut = r2;
-  }
-  return predict_mean_trunc_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r2cut, alpha, mean, work, stream);
+  return predict_mean_trunc_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, k->term, k->nterms, alpha, mean, work,
+                                   stream);
 }
 
 // ---- several outputs ----------------------------------------------------------------------------------------------
 // r is padded to R = 2, 4 or 8 accumulator columns; a one-term sum without white uses the single-term profile.
+// work == nullptr: the full sum; otherwise the truncated one with the cut-off of tgp_predict_mean_trunc_sum.
 template <int R, class Q>
 static int mean_multi_launch_r(const double* Xs, int64_t M, const double* X, int64_t N, const Q& prof, int r,
-                               double r2cut, const double* alpha, double* mean, double* work, void* stream) {
+                               const tgp_kernel_sum* k, const double* alpha, double* mean, double* work, void* stream) {
   const MultiOut<Q, R> mp{prof, r};
-  if (work) return predict_mean_trunc_launch(Xs, M, X, N, mp, r2cut, alpha, mean, work, stream);
+  if (work) return predict_mean_trunc_launch(Xs, M, X, N, mp, k->term, k->nterms, alpha, mean, work, stream);
   return predict_mean_launch(Xs, M, X, N, mp, alpha, mean, stream);
 }
 
 template <class Q>
 static int mean_multi_launch(const double* Xs, int64_t M, const double* X, int64_t N, const Q& prof, int r,
-                             double r2cut, const double* alpha, double* mean, double* work, void* stream) {
-  if (r <= 2) return mean_multi_launch_r<2>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
-  if (r <= 4) return mean_multi_launch_r<4>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
-  return mean_multi_launch_r<8>(Xs, M, X, N, prof, r, r2cut, alpha, mean, work, stream);
+                             const tgp_kernel_sum* k, const double* alpha, double* mean, double* work, void* stream) {
+  if (r <= 2) return mean_multi_launch_r<2>(Xs, M, X, N, prof, r, k, alpha, mean, work, stream);
+  if (r <= 4) return mean_multi_launch_r<4>(Xs, M, X, N, prof, r, k, alpha, mean, work, stream);
+  return mean_multi_launch_r<8>(Xs, M, X, N, prof, r, k, alpha, mean, work, stream);
 }
 
-// work == nullptr: the full sum; otherwise the truncated one with the cut-off of tgp_predict_mean_trunc_sum
-static int predict_mean_multi_impl(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
-                                   const double* alpha, int r, double* mean, double* work, void* stream) {
+static int mean_multi_entry(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
+                            const double* alpha, int r, double* mean, double* work, void* stream) {
   TGP_CHECK_ARG(r >= 1 && r <= TGP_MAX_RHS, "number of outputs must be 1 .. TGP_MAX_RHS");
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   if (r == 1)   // (N, 1) and (M, 1) are vectors: the single-output entries, bit for bit
     return work ? tgp_predict_mean_trunc_sum(Xs, M, X, N, k, alpha, mean, work, stream)
                 : tgp_predict_mean_sum(Xs, M, X, N, k, alpha, mean, stream);
-  TGP_CHECK_ARG(M >= 0 && N >= 0, "M/N");
-  if (M == 0) return TGP_OK;
-  TGP_CHECK_ARG(Xs && mean && (N == 0 || (X && alpha)), "null pointer");
-  if (N == 0) {
-    TGP_CUDA(cudaMemsetAsync(mean, 0, M * r * sizeof(double), (cudaStream_t)stream));
-    return TGP_OK;
-  }
-  double r2cut = 0.0;
-  if (work) {
-    for (int c = 0; c < k->nterms; ++c) {
-      const double lmin = metric_lmin(&k->term[c]);
-      TGP_CHECK_ARG(lmin > 0.0, "inverse metric must be positive definite");
-      const double r2 = profile_qcut(k->term[c].family) / lmin;
-      if (r2 > r2cut) r2cut = r2;
-    }
-  }
   if (k->nterms == 1) {
     const KDesc kd = make_kdesc(&k->term[0]);
-    TGP_FAMILY_SWITCH(k->term[0].family, return mean_multi_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, r, r2cut, alpha,
+    TGP_FAMILY_SWITCH(k->term[0].family, return mean_multi_launch(Xs, M, X, N, FamilyProfile<FAM>{kd}, r, k, alpha,
                                                                   mean, work, stream));
     return TGP_OK;
   }
-  return mean_multi_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r, r2cut, alpha, mean, work, stream);
+  return mean_multi_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, r, k, alpha, mean, work, stream);
 }
 
 extern "C" int tgp_predict_mean_multi(const double* Xs, int64_t M, const double* X, int64_t N, const tgp_kernel_sum* k,
                                       const double* alpha, int32_t r, double* mean, void* stream) {
-  return predict_mean_multi_impl(Xs, M, X, N, k, alpha, r, mean, nullptr, stream);
+  return mean_multi_entry(Xs, M, X, N, k, alpha, r, mean, nullptr, stream);
 }
 
 extern "C" int tgp_predict_mean_trunc_multi(const double* Xs, int64_t M, const double* X, int64_t N,
                                             const tgp_kernel_sum* k, const double* alpha, int32_t r, double* mean,
                                             double* work, void* stream) {
   TGP_CHECK_ARG(work != nullptr || M == 0 || N == 0, "work");
-  return predict_mean_multi_impl(Xs, M, X, N, k, alpha, r, mean, work, stream);
+  return mean_multi_entry(Xs, M, X, N, k, alpha, r, mean, work, stream);
 }
 
 // var[m] = amp - sum_n V[m][n]^2, V = K(Xs, X) L^-T (row m = L^-1 k*_m).  Warp per row.

@@ -306,6 +306,22 @@ extern "C" int tgp_loglike_grad(const double* X, const double* y, const double* 
   return TGP_OK;
 }
 
+// After the likelihood call of a sum: a one-term sum without white runs the single-term contraction (bit for bit the
+// single-term entry's gradient, d / d ln white = 0), any other sum its 4 nterms + 1 partial columns.
+static int grad_tail_sum(const double* X, int64_t N, const tgp_kernel_sum* k, double* work, int64_t ld,
+                         const double* alpha, double* out, const int32_t* info, const int64_t* row_end,
+                         double* scratch, cudaStream_t st, int nrhs) {
+  if (k->nterms == 1 && k->white == 0.0) {
+    TGP_CUDA(cudaMemsetAsync(out + 7, 0, sizeof(double), st));
+    const KDesc kd = make_kdesc(&k->term[0]);
+    TGP_FAMILY_SWITCH(k->term[0].family, return grad_tail(X, N, FamilyProfile<FAM>{kd}, 1, 4, work, ld, alpha, out,
+                                                          info, row_end, scratch, st, nrhs));
+    return TGP_OK;
+  }
+  return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
+                   row_end, scratch, st, nrhs);
+}
+
 extern "C" int tgp_loglike_grad_sum(const double* X, const double* y, const double* yerr2, int64_t N,
                                     const tgp_kernel_sum* k, double* work, int64_t ld, double* alpha, double* out,
                                     int32_t* info, const int64_t* row_end, int64_t nblocks, double* scratch,
@@ -313,15 +329,9 @@ extern "C" int tgp_loglike_grad_sum(const double* X, const double* y, const doub
   TGP_CHECK_ARG(ksum_ok(k), "kernel sum descriptor");
   int rc = grad_args(X, y, N, work, ld, alpha, out, info, row_end, nblocks, scratch);
   if (rc) return rc;
-  if (k->nterms == 1 && k->white == 0.0) {   // one term: the single-term entry bit for bit, d / d ln white = 0
-    TGP_CUDA(cudaMemsetAsync(out + 7, 0, sizeof(double), (cudaStream_t)stream));
-    return tgp_loglike_grad(X, y, yerr2, N, &k->term[0], work, ld, alpha, out, info, row_end, nblocks, scratch,
-                            stream);
-  }
   rc = tgp_loglike_sum(X, y, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream);
   if (rc) return rc;
-  return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
-                   row_end, scratch, (cudaStream_t)stream);
+  return grad_tail_sum(X, N, k, work, ld, alpha, out, info, row_end, scratch, (cudaStream_t)stream, 1);
 }
 
 extern "C" int tgp_loglike_grad_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
@@ -336,16 +346,7 @@ extern "C" int tgp_loglike_grad_multi(const double* X, const double* Y, int32_t 
     return tgp_loglike_grad_sum(X, Y, yerr2, N, k, work, ld, alpha, out, info, row_end, nblocks, scratch, stream);
   rc = tgp_loglike_multi(X, Y, r, yerr2, N, k, work, ld, alpha, 1, out, info, row_end, nblocks, stream);
   if (rc) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (k->nterms == 1 && k->white == 0.0) {   // one term: the single-term contraction, d / d ln white = 0
-    TGP_CUDA(cudaMemsetAsync(out + 7, 0, sizeof(double), st));
-    const KDesc kd = make_kdesc(&k->term[0]);
-    TGP_FAMILY_SWITCH(k->term[0].family, return grad_tail(X, N, FamilyProfile<FAM>{kd}, 1, 4, work, ld, alpha, out,
-                                                          info, row_end, scratch, st, r));
-    return TGP_OK;
-  }
-  return grad_tail(X, N, SumProfile{make_ksumdesc(k)}, k->nterms, 4 * k->nterms + 1, work, ld, alpha, out, info,
-                   row_end, scratch, st, r);
+  return grad_tail_sum(X, N, k, work, ld, alpha, out, info, row_end, scratch, (cudaStream_t)stream, r);
 }
 
 // ---- batches of independent problems (tgp_loglike_grad_batch) ---------------------------------------------------

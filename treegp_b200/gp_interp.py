@@ -148,7 +148,7 @@ class GPInterpolation(object):
         self._ensure_solved(self._y - self._mean - self._spatial_average, self._X, self.kernel, self._y_err)
         Xd, desc, ws = self._factor
         Xs = backend.as_points(X)
-        mean = self._predict_mean(Xs, Xd, desc)
+        mean = backend.predict_mean(Xs, Xd, desc, self._alpha_dev)
         var, self._var_plan = None, {}
         if self.WINDOWED_VARIANCE:
             var = backend.predict_var_windowed(Xs, Xd, desc, self._e2_dev, chunk=self.VAR_CHUNK, stats=self._var_plan)
@@ -158,48 +158,41 @@ class GPInterpolation(object):
         y = mean.cpu().numpy() + self._mean + self._build_average_meanify(X)
         return y, var.cpu().numpy()
 
-    def _predict_mean(self, Xs, Xd, desc):
-        """K(Xs, X) alpha on the device: (m,), or (m, r) for several outputs."""
-        if self._alpha_dev.dim() == 2:
-            return backend.predict_mean_multi(Xs, Xd, desc, self._alpha_dev)
-        return backend.predict_mean(Xs, Xd, desc, self._alpha_dev)
-
-    def _ensure_solved(self, y, X1, kernel, y_err):
-        """K + diag(y_err^2) -> L -> alpha on the device, cached like ``_alpha`` (gp_interp.py:179-182).  A y of
-        shape (n, r) gives alpha (n, r) from the same factorisation (tgp_loglike_multi)."""
-        if self._alpha is not None and self._factor is not None:
-            return
-        Xd = backend.as_points(X1)
-        n = Xd.shape[0]
-        desc = lower(kernel, Xd.shape[1])
-        e2 = backend.to_device(np.asarray(y_err, dtype=np.float64).reshape(-1) ** 2)
-        yd = _device_outputs(y)
-        # A kernel whose support is short against the field: with the points sorted along one axis K is zero (below
-        # 1e-40 amp) outside an envelope that its Cholesky factor keeps -- factorise inside it (N bw^2 flop instead of
-        # N^3 / 3).  The factor, X and alpha are then held in the sorted order; `_alpha` (host) in the caller's.
+    def _solve(self, Xd, yd, e2, desc):
+        """K + diag(e2) -> L -> alpha = K^-1 y on the device for y (n,) or (n, r).  A kernel whose support is short
+        against the field: with the points sorted along one axis K is zero (below 1e-40 amp) outside an envelope that
+        its Cholesky factor keeps -- factorise inside it (N bw^2 flop instead of N^3 / 3); X, y_err^2, alpha and the
+        factor are then in the sorted order.  Returns (X, y_err^2, alpha, workspace holding L, envelope plan or None);
+        raises as scipy.linalg.cholesky does (gp_interp.py:181) when K is not positive definite."""
         env = backend.plan_envelope(Xd, desc) if self.BANDED_SOLVE else None
         if env is not None:
             Xd, yd, e2 = Xd[env["order"]].contiguous(), yd[env["order"]].contiguous(), e2[env["order"]].contiguous()
-        # one call: K (lower) -> L with y riding through the factorisation as an extra row (forward substitution
-        # for free), then the backward sweep (tgp_loglike, want_alpha)
-        loglike = backend.loglike_multi if yd.dim() == 2 else backend.loglike
-        _, info, alpha, ws = loglike(Xd, yd, e2, desc, want_alpha=True, row_end=None if env is None else env["row_end"])
+        # one call: K (lower) -> L with y riding through the factorisation as extra rows (forward substitution
+        # for free), then the backward sweep (want_alpha)
+        _, info, alpha, ws = backend.loglike(Xd, yd, e2, desc, want_alpha=True,
+                                             row_end=None if env is None else env["row_end"])
         bad = int(info.item())
         if bad < 0:
             raise _cabi.TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % bad)
         if bad != 0:
-            # scipy.linalg.cholesky raises LinAlgError here (gp_interp.py:181)
             raise np.linalg.LinAlgError("%d-th leading minor of the array is not positive definite" % bad)
+        return Xd, e2, alpha, ws, env
+
+    def _ensure_solved(self, y, X1, kernel, y_err):
+        """K + diag(y_err^2) -> L -> alpha on the device, cached like ``_alpha`` (gp_interp.py:179-182).  A y of
+        shape (n, r) gives alpha (n, r) from the same factorisation.  With an envelope the factor, X and alpha are held
+        in the sorted order; `_alpha` (host) in the caller's."""
+        if self._alpha is not None and self._factor is not None:
+            return
+        Xd = backend.as_points(X1)
+        desc = lower(kernel, Xd.shape[1])
+        e2 = backend.to_device(np.asarray(y_err, dtype=np.float64).reshape(-1) ** 2)
+        Xd, e2, alpha, ws, env = self._solve(Xd, _device_outputs(y), e2, desc)
         self._factor = (Xd, desc, ws)
         self._e2_dev = e2        # y_err^2 in the order of Xd
         self._envelope = env
         self._alpha_dev = alpha
-        if env is None:
-            self._alpha = alpha.cpu().numpy()
-        else:
-            a = alpha.new_empty(alpha.shape)
-            a[env["order"]] = alpha
-            self._alpha = a.cpu().numpy()
+        self._alpha = (alpha if env is None else _unsort(alpha, env["order"])).cpu().numpy()
 
     def loo_predict(self):
         """Extension (not in the reference): leave-one-out predictions at every training point, in the caller's
@@ -217,25 +210,11 @@ class GPInterpolation(object):
         n = Xd.shape[0]
         desc = lower(self.kernel, Xd.shape[1])
         e2_host = np.asarray(self._y_err, dtype=np.float64).reshape(-1) ** 2
-        e2, yd = backend.to_device(e2_host), backend.to_device(y)
-        env = backend.plan_envelope(Xd, desc) if self.BANDED_SOLVE else None
-        if env is not None:
-            Xd, yd, e2 = Xd[env["order"]].contiguous(), yd[env["order"]].contiguous(), e2[env["order"]].contiguous()
-        row_end = None if env is None else env["row_end"]
-        loglike = backend.loglike_multi if multi else backend.loglike
-        _, info, alpha, ws = loglike(Xd, yd, e2, desc, want_alpha=True, row_end=row_end)
-        bad = int(info.item())
-        if bad < 0:
-            raise _cabi.TgpError("tgp_loglike: internal synchronisation timed out (info = %d)" % bad)
-        if bad != 0:
-            raise np.linalg.LinAlgError("%d-th leading minor of the array is not positive definite" % bad)
-        backend.selinv(ws, n, row_end=row_end)
+        _, _, alpha, ws, env = self._solve(Xd, backend.to_device(y), backend.to_device(e2_host), desc)
+        backend.selinv(ws, n, row_end=None if env is None else env["row_end"])
         zdiag = ws[:, :n].diagonal()
         if env is not None:
-            order = env["order"]
-            a, z = alpha.new_empty(alpha.shape), zdiag.new_empty(zdiag.shape)
-            a[order], z[order] = alpha, zdiag
-            alpha, zdiag = a, z
+            alpha, zdiag = _unsort(alpha, env["order"]), _unsort(zdiag, env["order"])
         alpha, zdiag = alpha.cpu().numpy(), zdiag.cpu().numpy()
         mean = y - alpha / (zdiag[:, None] if multi else zdiag) + self._mean + self._spatial_average
         return mean, 1.0 / zdiag - e2_host
@@ -248,7 +227,7 @@ class GPInterpolation(object):
         n = Xd.shape[0]
         Xs = backend.as_points(X2)
         m = Xs.shape[0]
-        y_predict = self._predict_mean(Xs, Xd, desc).cpu().numpy()
+        y_predict = backend.predict_mean(Xs, Xd, desc, self._alpha_dev).cpu().numpy()
         if not return_cov:
             return y_predict, None
         # y_cov = K** - K* (K + s^2 I)^-1 K*^T = K** - V V^T,  V = K* L^-T  (gp_interp.py:187-191)
@@ -387,6 +366,13 @@ class GPInterpolation(object):
                 plt.ylabel(r"$\Delta y$", fontsize=16)
             plt.title(title, fontsize=16)
         return fig
+
+
+def _unsort(t, order):
+    """The rows of t, which are in the order `order` of the caller's rows, back in the caller's order."""
+    u = t.new_empty(t.shape)
+    u[order] = t
+    return u
 
 
 def _device_outputs(y):

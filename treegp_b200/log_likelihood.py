@@ -84,12 +84,11 @@ class log_likelihood(object):
         if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf
         banded = self._envelope_inputs(desc)
-        loglike = backend.loglike_multi if yd.dim() == 2 else backend.loglike
         if banded is None:
-            out, info, _, _ = loglike(Xd, yd, e2, desc, work=work, want_alpha=False)
+            out, info, _, _ = backend.loglike(Xd, yd, e2, desc, work=work, want_alpha=False)
         else:
-            out, info, _, _ = loglike(banded[0], banded[1], banded[2], desc, work=work, want_alpha=False,
-                                      row_end=banded[3])
+            out, info, _, _ = backend.loglike(banded[0], banded[1], banded[2], desc, work=work, want_alpha=False,
+                                              row_end=banded[3])
             self.n_banded_evaluations = getattr(self, "n_banded_evaluations", 0) + 1
         self.n_evaluations += 1
         value = float(out[0].item())  # -inf when the matrix is not positive definite (info > 0)
@@ -111,12 +110,12 @@ class log_likelihood(object):
         if not np.all(np.isfinite(descriptor_params(desc))):
             return -np.inf, np.zeros(J.shape[1])
         banded = self._envelope_inputs(desc)
-        # several outputs: tgp_loglike_grad_multi, whose out has the sum layout (a single term's four derivatives first)
-        loglike_grad = backend.loglike_grad_multi if yd.dim() == 2 else backend.loglike_grad
+        # several outputs: out has the sum layout (a single term's four derivatives first)
         if banded is None:
-            out, info, _, _ = loglike_grad(Xd, yd, e2, desc, work=work)
+            out, info, _, _ = backend.loglike_grad(Xd, yd, e2, desc, work=work)
         else:
-            out, info, _, _ = loglike_grad(banded[0], banded[1], banded[2], desc, work=work, row_end=banded[3])
+            out, info, _, _ = backend.loglike_grad(banded[0], banded[1], banded[2], desc, work=work,
+                                                   row_end=banded[3])
             self.n_banded_evaluations = getattr(self, "n_banded_evaluations", 0) + 1
         self.n_evaluations += 1
         o = out.cpu().numpy()
