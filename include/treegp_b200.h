@@ -280,6 +280,28 @@ int64_t tgp_loglike_grad_batch_work_doubles(const int64_t* off /*host*/, int32_t
 int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off /*host*/,
                            int32_t B, const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, double* out,
                            int32_t* info, double* scratch, void* stream);
+/* vwork of tgp_predict_var_batch: sum_b min(M_b, chunk) ld_b doubles, M_b = soff[b+1] - soff[b]; -1 for invalid B,
+ * off, soff or chunk. */
+int64_t tgp_predict_var_batch_work_doubles(const int64_t* soff /*host*/, const int64_t* off /*host*/, int32_t B,
+                                           int64_t chunk);
+/* Diagonal predictive variance, rows [soff[b], soff[b+1]) of var for every problem, on the factors tgp_loglike_batch
+ * left in `work` (same off and ks): sum_c amp_c + white - |L_b^-1 k*|^2.  `chunk` (>= 1) test points per problem per
+ * pass; chunk, or the largest M_b if smaller, must not exceed min(65535 / ceil(max N_b / 64) * 128, 65535 * 64) so
+ * that every launch's grid stays within its limits.  vwork: tgp_predict_var_batch_work_doubles doubles, 16-byte
+ * aligned.  Equal bit for bit to tgp_predict_var_sum (row_end == NULL) on problem b's factor alone, for any chunk
+ * of either call. */
+int tgp_predict_var_batch(const double* Xs, const int64_t* soff /*host*/, const double* X, const int64_t* off /*host*/,
+                          int32_t B, const tgp_kernel_sum* ks /*host*/, const double* work, double* vwork,
+                          int64_t chunk, double* var, void* stream);
+/* Leave-one-out predictions of every problem: tgp_loglike_batch(want_alpha = 1), the selected inverse of
+ * tgp_loglike_grad_batch, then per training point the residual-space mean y_i - alpha_i / Z_ii and variance
+ * 1 / Z_ii - yerr2_i (loo_mean, loo_var: device double[off[B]]).  work, alpha and info as tgp_loglike_batch;
+ * scratch: tgp_loglike_grad_batch_work_doubles doubles, 16-byte aligned.  Rows of a problem with info != 0 are NaN.
+ * loo_var equals GPInterpolation.loo_predict on the dense factor bit for bit; loo_mean agrees to the rounding of
+ * alpha. */
+int tgp_loo_batch(const double* X, const double* y, const double* yerr2, const int64_t* off /*host*/, int32_t B,
+                  const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, double* scratch, double* loo_mean,
+                  double* loo_var, int32_t* info, void* stream);
 
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 

@@ -82,6 +82,9 @@ SIGNATURES = {
     "tgp_predict_mean_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp],
     "tgp_loglike_grad_batch_work_doubles": [_vp, _i32],
     "tgp_loglike_grad_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tgp_predict_var_batch_work_doubles": [_vp, _vp, _i32, _i64],
+    "tgp_predict_var_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp],
+    "tgp_loo_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -119,7 +122,7 @@ _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctyp
              "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
              "tgp_loglike_grad_multi_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64, "tgp_batch_work_doubles": ctypes.c_int64,
-             "tgp_loglike_grad_batch_work_doubles": ctypes.c_int64,
+             "tgp_loglike_grad_batch_work_doubles": ctypes.c_int64, "tgp_predict_var_batch_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 
 _lib = None

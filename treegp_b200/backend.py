@@ -454,6 +454,96 @@ def predict_mean_batch(Xs, ssizes, X, sizes, descs, alpha):
     return mean
 
 
+def var_batch_chunk_limit(sizes):
+    """The largest `chunk` tgp_predict_var_batch accepts for problems with `sizes` points: its gemm grid (row tiles of
+    128 times column tiles of 64 of the largest problem) and the K build's row tiles stay within 65535."""
+    return min(65535 // ((max(int(n) for n in sizes) + 63) // 64) * 128, 65535 * 64)
+
+
+def var_batch_chunk(ssizes, sizes, budget_bytes):
+    """Test points per problem per pass of tgp_predict_var_batch: the largest count whose V rows
+    (sum_b min(M_b, chunk) ld_b doubles) fit what `budget_bytes` leaves after the factors (batch_work_doubles(sizes)),
+    at least 1, at most max(M_b) and var_batch_chunk_limit(sizes).  Pure host function."""
+    m = np.asarray(ssizes, dtype=np.int64)
+    ld = (np.asarray(sizes, dtype=np.int64) + 1) & ~1
+    avail = budget_bytes - 8 * batch_work_doubles(sizes)
+    lo, hi = 1, max(1, min(int(m.max()) if len(m) else 1, var_batch_chunk_limit(sizes)))
+    while lo < hi:   # the V bytes grow with the chunk: the largest that fits
+        mid = (lo + hi + 1) // 2
+        if 8 * int(np.sum(np.minimum(m, mid) * ld)) <= avail:
+            lo = mid
+        else:
+            hi = mid - 1
+    return lo
+
+
+def predict_var_batch(Xs, ssizes, X, y, yerr2, sizes, descs, budget_bytes=4 << 30):
+    """Diagonal predictive variance of every problem (tgp_predict_var_batch), arguments as loglike_batch and
+    predict_mean_batch: rows [soff[b], soff[b+1]) are sum_c amp_c + white - |L_b^-1 k*|^2.  Each chunk of problems
+    (plan_batch_chunks) is factorised into a workspace of its own (tgp_loglike_batch, want_alpha = 0), then its test
+    points go through in passes of var_batch_chunk rows per problem; rows are solved independently, so the results
+    do not depend on either chunking.  Returns (var (sum M_b,), info (B,))."""
+    Xs, X = as_points(Xs), as_points(X)
+    sizes, ssizes = [int(n) for n in sizes], [int(m) for m in ssizes]
+    _check_batch_inputs(X, sizes, descs)
+    if len(ssizes) != len(sizes) or Xs.shape[0] != int(np.sum(ssizes)):
+        raise ValueError("need one test-point count per problem, adding up to the rows of Xs")
+    _check_dims(descs[0], X, Xs)
+    off, soff = batch_offsets(sizes), batch_offsets(ssizes)
+    B = len(sizes)
+    var = torch.empty(Xs.shape[0], dtype=F64, device=X.device)
+    info = torch.empty(B, dtype=torch.int32, device=X.device)
+    lib = _cabi.load()
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes):
+        r0, r1, s0, s1 = int(off[b0]), int(off[b1]), int(soff[b0]), int(soff[b1])
+        o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
+        so = np.ascontiguousarray(soff[b0:b1 + 1] - soff[b0])
+        ks = _ksum_array(descs[b0:b1])
+        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        alpha = torch.empty(r1 - r0, dtype=F64, device=X.device)
+        out = torch.empty((b1 - b0, 3), dtype=F64, device=X.device)
+        check(lib.tgp_loglike_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                    ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha), 0, _p(out),
+                                    _p(info[b0:b1]), _stream()), "tgp_loglike_batch")
+        if s1 == s0:
+            continue
+        chunk = var_batch_chunk(ssizes[b0:b1], sizes[b0:b1], budget_bytes)
+        nv = int(lib.tgp_predict_var_batch_work_doubles(_host_i64(so), _host_i64(o), b1 - b0, chunk))
+        check(min(nv, 0), "tgp_predict_var_batch_work_doubles")
+        vwork = torch.empty(nv, dtype=F64, device=X.device)
+        check(lib.tgp_predict_var_batch(_p(Xs[s0:s1]), _host_i64(so), _p(X[r0:r1]), _host_i64(o), b1 - b0,
+                                        ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(vwork), chunk, _p(var[s0:s1]),
+                                        _stream()), "tgp_predict_var_batch")
+    return var, info
+
+
+def loo_batch(X, y, yerr2, sizes, descs, budget_bytes=4 << 30):
+    """Leave-one-out predictions of every problem (tgp_loo_batch), arguments as loglike_batch, in chunks whose
+    workspace plus scratch fit `budget_bytes` (plan_batch_chunks(scratch=True)): mean_i = y_i - alpha_i / Z_ii and
+    var_i = 1 / Z_ii - yerr2_i in residual space, Z = K^-1.  Returns (mean, var, info): (sum N_b,), (sum N_b,), (B,);
+    the rows of a problem with info != 0 are NaN."""
+    X = as_points(X)
+    sizes = [int(n) for n in sizes]
+    _check_batch_inputs(X, sizes, descs)
+    off = batch_offsets(sizes)
+    B = len(sizes)
+    mean = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    var = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    info = torch.empty(B, dtype=torch.int32, device=X.device)
+    lib = _cabi.load()
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True):
+        r0, r1 = int(off[b0]), int(off[b1])
+        o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
+        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        scratch = torch.empty(grad_batch_scratch_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        alpha = torch.empty(r1 - r0, dtype=F64, device=X.device)
+        ks = _ksum_array(descs[b0:b1])
+        check(lib.tgp_loo_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha), _p(scratch), _p(mean[r0:r1]),
+                                _p(var[r0:r1]), _p(info[b0:b1]), _stream()), "tgp_loo_batch")
+    return mean, var, info
+
+
 TRUNC_MIN_M, TRUNC_MIN_N = 16384, 2048   # below this the plain kernel is launch-bound anyway
 
 

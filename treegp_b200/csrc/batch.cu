@@ -1,5 +1,6 @@
 // Batches of independent small problems: B likelihood evaluations (tgp_loglike_batch), B likelihoods with their
-// gradients (tgp_loglike_grad_batch) or B posterior means (tgp_predict_mean_batch) per call.
+// gradients (tgp_loglike_grad_batch), B posterior means (tgp_predict_mean_batch), B diagonal predictive variances
+// (tgp_predict_var_batch) or B sets of leave-one-out predictions (tgp_loo_batch) per call.
 //
 // A problem of a few hundred to a few thousand points leaves the B200 idle: its factorisation is a chain of small
 // launches (8 panel launches and one update per 512 columns, at most ~70 CTAs each), so its time is launch latency.
@@ -283,6 +284,28 @@ extern "C" int64_t tgp_loglike_grad_batch_work_doubles(const int64_t* off, int32
   return total;
 }
 
+// tgp_loglike_batch(want_alpha = 1) and the batched selected inverse on checked arguments.  T.extra holds
+// {logL, chi2, logdet} per problem, then the scratch block of every problem (*scr on the device), then `tail`.
+static int selinv_batch_run(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                            const tgp_kernel_sum* ks, double* work, double* alpha, int32_t* info, double* scratch,
+                            cudaStream_t st, BatchTables& T, std::vector<TgpBatchProb>& prob, double* const** scr,
+                            const std::vector<unsigned char>& tail = std::vector<unsigned char>()) {
+  const size_t o_scr = align16((size_t)B * 3 * sizeof(double));
+  const size_t o_tail = align16(o_scr + (size_t)B * sizeof(double*));
+  std::vector<unsigned char> extra(o_tail + tail.size(), 0);
+  if (!tail.empty()) memcpy(extra.data() + o_tail, tail.data(), tail.size());
+  double** scr_h = reinterpret_cast<double**>(extra.data() + o_scr);
+  int64_t soff = 0;
+  for (int32_t b = 0; b < B; ++b) {
+    scr_h[b] = scratch + soff;
+    soff += tgp_loglike_grad_sum_work_doubles(off[b + 1] - off[b], TGP_MAX_TERMS);
+  }
+  int rc = loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, 1, nullptr, info, st, T, prob, extra);
+  if (rc) return rc;
+  *scr = reinterpret_cast<double* const*>(T.extra + o_scr);
+  return tgp_batch_selinv(T.pr, *scr, prob.data(), scr_h, B, st);
+}
+
 extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off,
                                       int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, double* out,
                                       int32_t* info, double* scratch, void* stream) {
@@ -294,23 +317,12 @@ extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const do
   BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
   BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
-  // extra tables: {logL, chi2, logdet} per problem, then the scratch block of every problem
-  const size_t o_scr = align16((size_t)B * 3 * sizeof(double));
-  std::vector<unsigned char> extra(o_scr + (size_t)B * sizeof(double*), 0);
-  double** scr_h = reinterpret_cast<double**>(extra.data() + o_scr);
-  int64_t soff = 0;
-  for (int32_t b = 0; b < B; ++b) {
-    scr_h[b] = scratch + soff;
-    soff += tgp_loglike_grad_sum_work_doubles(off[b + 1] - off[b], TGP_MAX_TERMS);
-  }
   BatchTables T;
   std::vector<TgpBatchProb> prob;
-  rc = loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, 1, nullptr, info, st, T, prob, extra);
+  double* const* scr = nullptr;
+  rc = selinv_batch_run(X, y, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr);
   if (rc) return rc;
   const double* ll = reinterpret_cast<const double*>(T.extra);
-  double* const* scr = reinterpret_cast<double* const*>(T.extra + o_scr);
-  rc = tgp_batch_selinv(T.pr, scr, prob.data(), scr_h, B, st);
-  if (rc) return rc;
   for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
     if (T.start[c + 1] == T.start[c]) continue;
     int max_terms = 1;   // a sum's CTAs of terms beyond its own exit
@@ -356,6 +368,202 @@ extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, con
   for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
     if (T.start[c + 1] == T.start[c] || T.max_m[c] == 0) continue;
     rc = tgp_batch_predict_mean(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, T.max_m[c], st);
+    if (rc) return rc;
+  }
+  return TGP_OK;
+}
+
+// ---- leave-one-out predictions (tgp_loo_batch) ---------------------------------------------------------------------
+// One CTA per problem, in residual space, with the operations of GPInterpolation.loo_predict in the same order:
+// mean_i = y_i - alpha_i / Z_ii, var_i = 1 / Z_ii - yerr2_i; NaN for a problem with info != 0.
+__global__ void __launch_bounds__(256)
+loo_finish_batch_kernel(const TgpBatchProb* __restrict__ pr, const int64_t* __restrict__ off,
+                        const int32_t* __restrict__ info, double* __restrict__ mean, double* __restrict__ var) {
+  const TgpBatchProb& p = pr[blockIdx.x];
+  const int64_t r0 = off[blockIdx.x];
+  const bool ok = info[blockIdx.x] == 0;
+  const double nan = __longlong_as_double(0x7ff8000000000000ll);
+  for (int64_t i = threadIdx.x; i < p.N; i += blockDim.x) {
+    const double z = p.A[i * p.ld + i];
+    mean[r0 + i] = ok ? p.y[i] - p.alpha[i] / z : nan;
+    var[r0 + i] = ok ? 1.0 / z - p.yerr2[i] : nan;
+  }
+}
+
+extern "C" int tgp_loo_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                             const tgp_kernel_sum* ks, double* work, double* alpha, double* scratch, double* loo_mean,
+                             double* loo_var, int32_t* info, void* stream) {
+  const char* fn = __func__;
+  int rc = check_batch(fn, off, B, ks);
+  if (rc) return rc;
+  BATCH_CHECK(X && y && yerr2 && work && alpha && scratch && loo_mean && loo_var && info,
+              "null pointer (X, y, yerr2, work, alpha, scratch, loo_mean, loo_var, info)");
+  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
+  BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<unsigned char> tail((size_t)(B + 1) * sizeof(int64_t));   // the offsets, for the finish
+  memcpy(tail.data(), off, tail.size());
+  BatchTables T;
+  std::vector<TgpBatchProb> prob;
+  double* const* scr = nullptr;
+  rc = selinv_batch_run(X, y, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr, tail);
+  if (rc) return rc;
+  const int64_t* off_d = reinterpret_cast<const int64_t*>(reinterpret_cast<const unsigned char*>(scr) +
+                                                          align16((size_t)B * sizeof(double*)));
+  loo_finish_batch_kernel<<<(unsigned)B, 256, 0, st>>>(T.pr, off_d, info, loo_mean, loo_var);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// ---- predictive variance (tgp_predict_var_batch) -------------------------------------------------------------------
+// Per pass over `chunk` test points of every problem: K(Xs, X) into each problem's rows of vwork, then V <- V L^-T as
+// trsm_rows_blocked (dense) runs it, for all problems in one launch sequence: per 512-wide block column of the largest
+// problem the halving solve (leaf, gemm, leaf, ..., the gemm between leaves i and i + 1 shaped by tgp_halving_node) and
+// the trailing update V[:, c1:N] -= V[:, k:c1] L[c1:N, k:c1]^T; last the variance of every row.  Every launch runs the
+// single-problem body with the single call's operands, so each row gets tgp_predict_var_sum's arithmetic.
+
+// The largest row count per pass the launches accept: the gemm grid (row tiles x column tiles) and the K build's row
+// tiles stay within 65535.
+static int64_t var_chunk_limit(int64_t max_n) { return std::min<int64_t>(65535 / tgp_cdiv(max_n, 64) * 128, 65535 * 64); }
+
+static int check_var_batch(const char* fn, const int64_t* soff, const int64_t* off, int32_t B, int64_t chunk) {
+  BATCH_CHECK(B >= 1, "B must be >= 1");
+  int rc = check_offsets(fn, "off", off, B, 1, TGP_BATCH_MAX_N);
+  if (rc) return rc;
+  rc = check_offsets(fn, "soff", soff, B, 0, INT64_MAX);
+  if (rc) return rc;
+  BATCH_CHECK(chunk >= 1, "chunk must be >= 1");
+  int64_t max_n = 0, max_m = 0;
+  for (int32_t b = 0; b < B; ++b) {
+    max_n = std::max(max_n, off[b + 1] - off[b]);
+    max_m = std::max(max_m, soff[b + 1] - soff[b]);
+  }
+  char msg[160];
+  snprintf(msg, sizeof msg, "chunk = %lld exceeds %lld test points per pass (grid limit for N_b = %lld)",
+           (long long)chunk, (long long)var_chunk_limit(max_n), (long long)max_n);
+  BATCH_CHECK(std::min(chunk, max_m) <= var_chunk_limit(max_n), msg);
+  return TGP_OK;
+}
+
+extern "C" int64_t tgp_predict_var_batch_work_doubles(const int64_t* soff, const int64_t* off, int32_t B,
+                                                      int64_t chunk) {
+  if (check_var_batch(__func__, soff, off, B, chunk)) return TGP_ERR_INVALID;
+  int64_t total = 0;
+  for (int32_t b = 0; b < B; ++b) total += std::min(soff[b + 1] - soff[b], chunk) * even_ld(off[b + 1] - off[b]);
+  return total;
+}
+
+struct VarOp {   // one launch of the row solve: the leaves of one halving step, or one gemm
+  std::vector<TgpLeafArgs> full, edge;
+  std::vector<TgpGemmArgs> gemm;
+};
+
+extern "C" int tgp_predict_var_batch(const double* Xs, const int64_t* soff, const double* X, const int64_t* off,
+                                     int32_t B, const tgp_kernel_sum* ks, const double* work, double* vwork,
+                                     int64_t chunk, double* var, void* stream) {
+  const char* fn = __func__;
+  int rc = check_var_batch(fn, soff, off, B, chunk);
+  if (rc) return rc;
+  rc = check_batch(fn, off, B, ks);
+  if (rc) return rc;
+  BATCH_CHECK(X && work, "null pointer (X, work)");
+  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
+  if (soff[B] == 0) return TGP_OK;
+  BATCH_CHECK(Xs && vwork && var, "null pointer (Xs, vwork, var)");
+  BATCH_CHECK(((uintptr_t)vwork & 15) == 0, "vwork must be 16-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  const int ndim = ks[0].ndim;
+  std::vector<int> cls(B);
+  std::vector<int64_t> Nh(B), ld(B), voff(B), woff(B);
+  std::vector<double> prior(B);
+  int64_t max_n = 0, max_m = 0, v = 0, w = 0;
+  for (int32_t b = 0; b < B; ++b) {
+    Nh[b] = off[b + 1] - off[b];
+    ld[b] = even_ld(Nh[b]);
+    woff[b] = w;
+    w += (Nh[b] + 1) * ld[b];
+    voff[b] = v;
+    v += std::min(soff[b + 1] - soff[b], chunk) * ld[b];
+    max_n = std::max(max_n, Nh[b]);
+    max_m = std::max(max_m, soff[b + 1] - soff[b]);
+    // tgp_kmat_cross_sum: the single-term kernel for any one-term sum (no white term in K(Xs, X))
+    cls[b] = ks[b].nterms == 1 ? ks[b].term[0].family : TGP_BATCH_SUM;
+    double p = ks[b].white;   // the prior variance in predict_var_impl's order
+    for (int c = 0; c < ks[b].nterms; ++c) p += ks[b].term[c].amp;
+    prior[b] = p;
+  }
+  for (int64_t m0 = 0; m0 < max_m; m0 += chunk) {
+    std::vector<TgpBatchProb> prob(B);
+    std::vector<int64_t> mc(B);
+    for (int32_t b = 0; b < B; ++b) {
+      TgpBatchProb& p = prob[b];
+      p = TgpBatchProb{};
+      mc[b] = std::max<int64_t>(0, std::min(soff[b + 1] - soff[b] - m0, chunk));
+      p.X = X + off[b] * ndim;
+      p.N = Nh[b];
+      p.ld = ld[b];
+      p.A = vwork + voff[b];
+      p.M = mc[b];
+      p.Xs = Xs + (soff[b] + (mc[b] ? m0 : 0)) * ndim;
+      p.mean = var + soff[b] + (mc[b] ? m0 : 0);
+    }
+    // the launch sequence of the row solve
+    std::vector<VarOp> ops;
+    for (int64_t k = 0; k < max_n; k += TGP_OB) {
+      int64_t wmax = 0;
+      for (int32_t b = 0; b < B; ++b)
+        if (mc[b] > 0 && Nh[b] > k) wmax = std::max(wmax, std::min<int64_t>(TGP_OB, Nh[b] - k));
+      const int nleaves = (int)tgp_cdiv(wmax, 64);
+      for (int i = 0; i < nleaves; ++i) {
+        ops.emplace_back();
+        const int64_t c0 = 64 * (int64_t)i;
+        for (int32_t b = 0; b < B; ++b) {   // leaf i of problem b, on the path trsm_panel_launch takes for it
+          const int64_t wb = std::min<int64_t>(TGP_OB, Nh[b] - k);
+          if (mc[b] == 0 || wb <= c0) continue;
+          const double* L = work + woff[b] + (k + c0) * ld[b] + k + c0;
+          double* Vb = prob[b].A + k + c0;
+          const int nb = (int)std::min<int64_t>(wb - c0, 64);
+          const bool full = nb == 64 && (ld[b] & 1) == 0 && ((uintptr_t)Vb & 15) == 0;
+          (full ? ops.back().full : ops.back().edge).push_back(TgpLeafArgs{L, Vb, ld[b], mc[b], ld[b], nb});
+        }
+        if (i + 1 == nleaves) break;
+        ops.emplace_back();
+        for (int32_t b = 0; b < B; ++b) {   // B2 -= B1 L21^T on the node [o, o + n) of leaves i and i + 1, split at h
+          const int64_t wb = std::min<int64_t>(TGP_OB, Nh[b] - k);
+          if (mc[b] == 0 || wb <= 0 || i + 1 >= tgp_cdiv(wb, 64)) continue;
+          int64_t o, h, n;
+          tgp_halving_node(wb, i, o, h, n);
+          const double* Lk = work + woff[b] + k * ld[b] + k;
+          double* Vk = prob[b].A + k;
+          ops.back().gemm.push_back(TgpGemmArgs{Vk + o + h, Vk + o, Lk + (o + h) * ld[b] + o, mc[b], n - h, h, ld[b]});
+        }
+      }
+      ops.emplace_back();
+      const int64_t c1 = k + TGP_OB;
+      for (int32_t b = 0; b < B; ++b) {   // V[:, c1:N] -= V[:, k:c1] L[c1:N, k:c1]^T
+        if (mc[b] == 0 || Nh[b] <= c1) continue;
+        ops.back().gemm.push_back(TgpGemmArgs{prob[b].A + c1, prob[b].A + k, work + woff[b] + c1 * ld[b] + k, mc[b],
+                                              Nh[b] - c1, TGP_OB, ld[b]});
+      }
+    }
+    std::vector<unsigned char> extra((size_t)B * sizeof(double));   // the prior variances
+    memcpy(extra.data(), prior.data(), extra.size());
+    BatchTables T;
+    rc = stage_tables(T, prob, ks, cls, st, extra);
+    if (rc) return rc;
+    for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
+      if (T.start[c + 1] == T.start[c] || T.max_m[c] == 0) continue;
+      rc = tgp_batch_kmat_cross(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, T.max_n[c],
+                                T.max_m[c], st);
+      if (rc) return rc;
+    }
+    for (const VarOp& op : ops) {
+      if ((rc = tgp_batch_gemm(op.gemm.data(), (int32_t)op.gemm.size(), st))) return rc;
+      if ((rc = tgp_batch_selinv_leaves(op.full.data(), (int32_t)op.full.size(), true, st))) return rc;
+      if ((rc = tgp_batch_selinv_leaves(op.edge.data(), (int32_t)op.edge.size(), false, st))) return rc;
+    }
+    rc = tgp_batch_var_rows(T.pr, reinterpret_cast<const double*>(T.extra), B,
+                            std::min(chunk, max_m - m0), st);
     if (rc) return rc;
   }
   return TGP_OK;

@@ -1,4 +1,5 @@
-// Batches of independent problems (tgp_loglike_batch, tgp_loglike_grad_batch, tgp_predict_mean_batch): the per-problem
+// Batches of independent problems (tgp_loglike_batch, tgp_loglike_grad_batch, tgp_predict_mean_batch,
+// tgp_predict_var_batch, tgp_loo_batch): the per-problem
 // table the batched kernels read, and the launchers that kmat.cu, dense.cu, selinv.cu and predict.cu provide to
 // batch.cu.  Every batched kernel
 // runs the body of its single-problem twin on one problem's slice, so each problem gets the single call's arithmetic.
@@ -131,6 +132,26 @@ struct TgpLeafLaunch {
 int tgp_batch_selinv_leaves(const TgpLeafArgs* leaves, int32_t n, bool full, cudaStream_t st);
 int tgp_batch_selinv_gemm(const TgpBatchProb* pr, double* const* scr, int32_t B, int s, int op, int leaf,
                           int tiles_n, int64_t tiles, cudaStream_t st);
+// ---- predictive variance of a batch (tgp_predict_var_batch) --------------------------------------------------------
+// K(Xs_b, X_b) into the pr[b].M x pr[b].ld rows at pr[b].A for the problems `list` (profile class of tgp_kmat_cross_sum).
+int tgp_batch_kmat_cross(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
+                         int64_t max_n, int64_t max_m, cudaStream_t st);
+// One C (M x Nc) -= A B^T with inner dimension Kd per entry, launched as gemm_nt_sub_kernel's tiles.  The entries
+// travel in the parameter bank, as the leaves' do: read from global memory they would spill the tile's registers.
+struct TgpGemmArgs {
+  double* C;
+  const double* A;
+  const double* B;
+  int64_t M, Nc, Kd, ld;   // C, A and B share the row pitch ld
+};
+constexpr int TGP_GEMM_GROUP = 256;   // entries per launch (14 KB)
+struct TgpGemmLaunch {
+  TgpGemmArgs a[TGP_GEMM_GROUP];
+};
+int tgp_batch_gemm(const TgpGemmArgs* entries, int32_t n, cudaStream_t st);   // n entries (host array), all M > 0
+// pr[b].mean[m] = prior[b] - sum_n V_b[m, n]^2 for the pr[b].M rows V_b at pr[b].A (var_from_rows_kernel's body).
+int tgp_batch_var_rows(const TgpBatchProb* pr, const double* prior, int32_t B, int64_t max_m, cudaStream_t st);
+
 // The contraction of the problems `list` (profile class cls) into their scratch, then one finishing CTA per problem
 // writing out[b * TGP_GRAD_BATCH_OUT ..] from ll[3 b ..] = {logL, chi2, logdet}, the tile sums and info.
 int tgp_batch_grad_contract(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,

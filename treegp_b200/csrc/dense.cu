@@ -1475,3 +1475,37 @@ int tgp_batch_selinv_gemm(const TgpBatchProb* pr, double* const* scr, int32_t B,
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }
+
+// grid: (entry, row tile * tiles_n + column tile): gemm_nt_sub_kernel's tile of entry blockIdx.x (the batched row solve
+// of tgp_predict_var_batch); tiles outside an entry's product exit.
+__global__ void __launch_bounds__(GEMM_THREADS, 2)
+gemm_batch_kernel(const __grid_constant__ TgpGemmLaunch p, int tiles_n) {
+  const TgpGemmArgs& a = p.a[blockIdx.x];
+  const int64_t m0 = (int64_t)(blockIdx.y / tiles_n) * BM, n0 = (int64_t)(blockIdx.y % tiles_n) * 64;
+  if (m0 >= a.M || n0 >= a.Nc) return;
+  gemm_nt_sub_tile<64, 4, 2>(a.C, a.M, a.Nc, a.ld, a.A, a.ld, a.B, a.ld, a.Kd, 0, m0, n0);
+}
+
+int tgp_batch_gemm(const TgpGemmArgs* entries, int32_t n, cudaStream_t st) {
+  constexpr int GSMEM = STAGES * (BM + 64) * BK * 8;
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once)) {
+    TGP_CUDA(cudaFuncSetAttribute(gemm_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GSMEM));
+    TGP_CUDA(cudaFuncSetAttribute(gemm_batch_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
+  }
+  for (int32_t i0 = 0; i0 < n; i0 += TGP_GEMM_GROUP) {
+    TgpGemmLaunch p;
+    const int32_t cnt = std::min(n - i0, TGP_GEMM_GROUP);
+    int64_t tm = 0, tn = 0;
+    for (int32_t i = 0; i < cnt; ++i) {
+      p.a[i] = entries[i0 + i];
+      tm = std::max(tm, tgp_cdiv(p.a[i].M, BM));
+      tn = std::max(tn, tgp_cdiv(p.a[i].Nc, 64));
+    }
+    TGP_CHECK_ARG(tm * tn <= 65535, "too many tiles for one launch");
+    gemm_batch_kernel<<<dim3((unsigned)cnt, (unsigned)(tm * tn)), GEMM_THREADS, GSMEM, st>>>(p, (int)tn);
+    TGP_LAUNCH_CHECK();
+  }
+  return TGP_OK;
+}

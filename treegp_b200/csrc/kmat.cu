@@ -159,15 +159,15 @@ kmat_sym_kernel(const double* __restrict__ X, int64_t N, P prof, const double* _
   kmat_sym_tile(X, N, prof, diag_add, out, ld, lower_only, vec_ok, phi_g, (int64_t)blockIdx.x);
 }
 
-// Rectangular build K(Xs, X): rows = test points, columns = training points.
+// Rectangular build K(Xs, X): rows = test points, columns = training points.  The tile whose top-left corner is
+// (r0, c0).
 template <class P>
-__global__ void __launch_bounds__(KT_THREADS)
-kmat_cross_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
-                  P prof, double* __restrict__ out, int64_t ld, int vec_ok,
-                  const double* __restrict__ phi_g) {
+__device__ __forceinline__ void kmat_cross_tile(const double* __restrict__ Xs, int64_t M,
+                                                const double* __restrict__ X, int64_t N, const P& prof,
+                                                double* __restrict__ out, int64_t ld, int vec_ok,
+                                                const double* __restrict__ phi_g, const int64_t r0, const int64_t c0) {
   __shared__ double xr[KT], yr[KT], xc[KT], yc[KT];
   __shared__ double phi_s[P::kPhiSize];
-  const int64_t r0 = (int64_t)blockIdx.x * KT, c0 = (int64_t)blockIdx.y * KT;
   const int tid = threadIdx.x;
   if (prof.stage_phi()) tgp_stage_phi(phi_s, phi_g);
   if (tid < KT) {
@@ -198,6 +198,14 @@ kmat_cross_kernel(const double* __restrict__ Xs, int64_t M, const double* __rest
     const bool ok0 = cg < N, ok1 = cg + 1 < N;
     store2(out + rg * ld + cg, v0, v1, vec_ok && ok0, ok0, ok1);
   }
+}
+
+template <class P>
+__global__ void __launch_bounds__(KT_THREADS)
+kmat_cross_kernel(const double* __restrict__ Xs, int64_t M, const double* __restrict__ X, int64_t N,
+                  P prof, double* __restrict__ out, int64_t ld, int vec_ok,
+                  const double* __restrict__ phi_g) {
+  kmat_cross_tile(Xs, M, X, N, prof, out, ld, vec_ok, phi_g, (int64_t)blockIdx.x * KT, (int64_t)blockIdx.y * KT);
 }
 
 // ---- C ABI -----------------------------------------------------------------------------------
@@ -290,6 +298,48 @@ int tgp_batch_kmat_sym(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t
     kmat_sym_batch_kernel<SumProfile><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi);
   } else {
     TGP_FAMILY_SWITCH(cls, (kmat_sym_batch_kernel<FamilyProfile<FAM>><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi)));
+  }
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// K(Xs_b, X_b) into the M x ld rows at pr[b].A (tgp_predict_var_batch).  Grid: (problems of this profile class, column
+// tiles, row tiles of the largest of them); each CTA runs the tile body of the single build.  A sum's profile is staged
+// in shared memory: its terms are indexed at run time, which a copy in registers could only do from the stack.  A
+// family's profile stays in registers, as in the single build: read from shared memory, its quadratic form compiles to
+// a different contraction of products into FMAs, and K differs from the single build in the last bit.
+template <class P>
+__global__ void __launch_bounds__(KT_THREADS)
+kmat_cross_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* __restrict__ kd,
+                        const int32_t* __restrict__ list, const double* __restrict__ phi_g) {
+  const int b = list[blockIdx.x];
+  const int64_t M = pr[b].M, N = pr[b].N, r0 = (int64_t)blockIdx.z * KT, c0 = (int64_t)blockIdx.y * KT;
+  if (r0 >= M || c0 >= N) return;
+  if constexpr (P::kSum) {
+    __shared__ P prof_s;
+    static_assert(sizeof(prof_s.desc) == sizeof(P) && sizeof(P) % 4 == 0, "a profile is its descriptor");
+    const int* src = reinterpret_cast<const int*>(&kd[b]);
+    int* dst = reinterpret_cast<int*>(&prof_s);
+    for (int i = threadIdx.x; i < (int)(sizeof(P) / 4); i += KT_THREADS) dst[i] = src[i];
+    __syncthreads();
+    kmat_cross_tile(pr[b].Xs, M, pr[b].X, N, prof_s, pr[b].A, pr[b].ld, /*vec_ok=*/1, phi_g, r0, c0);
+  } else {
+    const P prof = tgp_batch_profile<P>(kd[b]);
+    kmat_cross_tile(pr[b].Xs, M, pr[b].X, N, prof, pr[b].A, pr[b].ld, /*vec_ok=*/1, phi_g, r0, c0);
+  }
+}
+
+int tgp_batch_kmat_cross(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
+                         int64_t max_n, int64_t max_m, cudaStream_t st) {
+  const int64_t rt = tgp_cdiv(max_m, KT);
+  TGP_CHECK_ARG(rt <= 65535, "too many test points per problem in one pass");
+  const dim3 grid((unsigned)count, (unsigned)tgp_cdiv(max_n, KT), (unsigned)rt);
+  const double* phi = tgp_phi_device();
+  if (cls == TGP_BATCH_SUM) {
+    kmat_cross_batch_kernel<SumProfile><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi);
+  } else {
+    TGP_FAMILY_SWITCH(cls,
+                      (kmat_cross_batch_kernel<FamilyProfile<FAM>><<<grid, KT_THREADS, 0, st>>>(pr, kd, list, phi)));
   }
   TGP_LAUNCH_CHECK();
   return TGP_OK;

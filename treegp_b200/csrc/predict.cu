@@ -465,22 +465,28 @@ extern "C" int tgp_predict_mean_trunc_multi(const double* Xs, int64_t M, const d
 __global__ void __launch_bounds__(256)
 var_from_rows_kernel(const double* __restrict__ V, int64_t M, int64_t N, int64_t ldv, double amp,
                      double* __restrict__ var) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int64_t m = (int64_t)blockIdx.x * 8 + warp;
-  if (m >= M) return;
-  const double* row = V + m * ldv;
-  double s0 = 0.0, s1 = 0.0;
-  int64_t n = lane;
-  for (; n + 32 < N; n += 64) {
-    const double a = row[n], b = row[n + 32];
-    s0 = fma(a, a, s0);
-    s1 = fma(b, b, s1);
+#include "var_rows_body.cuh"
+}
+
+// grid: (warp-row block of the largest problem, problem b0 + blockIdx.y)
+__global__ void __launch_bounds__(256)
+var_rows_batch_kernel(const TgpBatchProb* __restrict__ pr, const double* __restrict__ prior, int32_t b0) {
+  const TgpBatchProb& p = pr[b0 + blockIdx.y];
+  const double* const V = p.A;
+  const int64_t M = p.M, N = p.N, ldv = p.ld;
+  const double amp = prior[b0 + blockIdx.y];
+  double* const var = p.mean;
+#include "var_rows_body.cuh"
+}
+
+int tgp_batch_var_rows(const TgpBatchProb* pr, const double* prior, int32_t B, int64_t max_m, cudaStream_t st) {
+  const int64_t gx = tgp_cdiv(max_m, 8);
+  TGP_CHECK_ARG(gx < (1ll << 31), "too many test points per problem in one pass");
+  for (int32_t b0 = 0; b0 < B; b0 += 65535) {   // gridDim.y <= 65535
+    var_rows_batch_kernel<<<dim3((unsigned)gx, (unsigned)std::min(B - b0, 65535)), 256, 0, st>>>(pr, prior, b0);
+    TGP_LAUNCH_CHECK();
   }
-  if (n < N) { const double a = row[n]; s0 = fma(a, a, s0); }
-  double s = s0 + s1;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (lane == 0) var[m] = amp - s;
+  return TGP_OK;
 }
 
 // k or ks (the other NULL): single-term or sum kernel; the prior variance is amp, or sum_c amp_c + white

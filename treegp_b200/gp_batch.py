@@ -257,25 +257,45 @@ class GPInterpolationBatch(object):
                               robust_fit=self.optimizer == "anisotropic", p0=self.p0_robust_fit)
                 self.kernels[b] = fit.optimizer(self.kernels[b])
 
-    def _ensure_solved(self):
-        """alpha = K^-1 y of every problem for the current kernels (one batched call), cached until the next fit."""
-        if self._solved is not None:
-            return self._solved
-        X, y, e2, sizes, _ = self._device_data()
-        descs = [lower(k, X.shape[1]) for k in self.kernels]
+    def _descriptors(self):
+        """Every problem's kernel descriptor; LinAlgError naming the first problem whose kernel is not finite."""
+        ndim = self._X[0].shape[1]
+        descs = [lower(k, ndim) for k in self.kernels]
         for b, d in enumerate(descs):
             if not np.all(np.isfinite(descriptor_params(d))):
                 raise np.linalg.LinAlgError("problem %d: the kernel has non-finite parameters" % b)
-        _, info, alpha = backend.loglike_batch(X, y, e2, sizes, descs, want_alpha=True, budget_bytes=self.WORK_BUDGET)
+        return descs
+
+    @staticmethod
+    def _raise_on_info(info, name):
+        """TgpError for info < 0, LinAlgError naming the first problem whose K is not positive definite."""
         info = info.cpu().numpy()
         if np.any(info < 0):
-            raise _cabi.TgpError("tgp_loglike_batch: internal synchronisation timed out (info = %r)" % info.tolist())
+            raise _cabi.TgpError("%s: internal synchronisation timed out (info = %r)" % (name, info.tolist()))
         bad = np.flatnonzero(info > 0)
         if len(bad):
             raise np.linalg.LinAlgError("problem %d: %d-th leading minor of the array is not positive definite"
                                         % (bad[0], info[bad[0]]))
+
+    def _ensure_solved(self):
+        """alpha = K^-1 y of every problem for the current kernels (one batched call), cached until the next fit."""
+        if self._solved is not None:
+            return self._solved
+        descs = self._descriptors()
+        X, y, e2, sizes, _ = self._device_data()
+        _, info, alpha = backend.loglike_batch(X, y, e2, sizes, descs, want_alpha=True, budget_bytes=self.WORK_BUDGET)
+        self._raise_on_info(info, "tgp_loglike_batch")
         self._solved = (descs, alpha)
         return self._solved
+
+    def _check_positions(self, Xs_new):
+        """ValueError, before any device work, unless Xs_new holds one (M_b, ndim) array per problem."""
+        if len(Xs_new) != len(self._X):
+            raise ValueError("need one set of positions per problem (%d for %d problems)" % (len(Xs_new), len(self._X)))
+        ndim = self._X[0].shape[1]
+        for b, x in enumerate(Xs_new):
+            if np.ndim(x) != 2 or np.shape(x)[1] != ndim:
+                raise ValueError("problem %d: positions must have shape (M, %d); got %r" % (b, ndim, np.shape(x)))
 
     def predict(self, Xs_new, return_cov=False):
         """Posterior means at the positions Xs_new[b] (M_b, ndim) of every problem: a list of B arrays."""
@@ -290,6 +310,37 @@ class GPInterpolationBatch(object):
         mean = backend.predict_mean_batch(Xs, ssizes, X, sizes, descs, alpha).cpu().numpy()
         soff = backend.batch_offsets(ssizes)
         return [mean[soff[b]:soff[b + 1]] + self._mean[b] + np.zeros(ssizes[b]) for b in range(len(sizes))]
+
+    def predict_var(self, Xs_new):
+        """Posterior means and DIAGONAL predictive variances at the positions Xs_new[b] (M_b, ndim) of every problem:
+        (means, vars), two lists of B arrays.  The means are predict's; the variances are what
+        GPInterpolation.predict_var returns for the problem, bit for bit with its dense solve (residual space: the
+        normalising mean does not enter).  All problems' test points go through one batched call
+        (tgp_predict_var_batch), which factorises into a workspace of its own."""
+        self._check_positions(Xs_new)
+        means = self.predict(Xs_new)
+        descs, _ = self._ensure_solved()
+        X, y, e2, sizes, _ = self._device_data()
+        ssizes = [len(m) for m in means]
+        Xs = torch.cat([backend.as_points(x) for x in Xs_new])
+        var, info = backend.predict_var_batch(Xs, ssizes, X, y, e2, sizes, descs, budget_bytes=self.WORK_BUDGET)
+        self._raise_on_info(info, "tgp_loglike_batch")
+        var = var.cpu().numpy()
+        soff = backend.batch_offsets(ssizes)
+        return means, [var[soff[b]:soff[b + 1]] for b in range(len(sizes))]
+
+    def loo_predict(self):
+        """Leave-one-out predictions at every training point of every problem, without refitting: (means, vars), two
+        lists of B arrays in each problem's own order, as GPInterpolation.loo_predict gives them -- mean_i = y_i -
+        alpha_i / Z_ii plus the normalising mean, var_i = 1 / Z_ii - y_err_i^2, Z = (K + diag(y_err^2))^-1.  One
+        batched call (tgp_loo_batch) factorises and inverts every problem in a workspace of its own."""
+        descs = self._descriptors()
+        X, y, e2, sizes, off = self._device_data()
+        mean, var, info = backend.loo_batch(X, y, e2, sizes, descs, budget_bytes=self.WORK_BUDGET)
+        self._raise_on_info(info, "tgp_loo_batch")
+        mean, var = mean.cpu().numpy(), var.cpu().numpy()
+        return ([mean[off[b]:off[b + 1]] + self._mean[b] + self._spatial_average[b] for b in range(len(sizes))],
+                [var[off[b]:off[b + 1]] for b in range(len(sizes))])
 
     def return_log_likelihood(self, thetas=None):
         """Marginal log-likelihood of every problem for its current kernel, or for thetas[b] if given: an array of B
