@@ -302,6 +302,35 @@ int tgp_predict_var_batch(const double* Xs, const int64_t* soff /*host*/, const 
 int tgp_loo_batch(const double* X, const double* y, const double* yerr2, const int64_t* off /*host*/, int32_t B,
                   const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, double* scratch, double* loo_mean,
                   double* loo_var, int32_t* info, void* stream);
+/* Several outputs per problem (1 <= r <= TGP_MAX_RHS, one r for the whole batch), sharing its kernel and its
+ * factorisation as in tgp_loglike_multi: Y, alpha (and loo_mean) are row-major (sum N_b) x r with problem b owning
+ * rows [off[b], off[b+1]); yerr2 stays (sum N_b,), shared by the outputs; mean is (sum M_b) x r.  Arguments are those
+ * of the single-output entries plus r, checked before any CUDA call, and with r == 1 each entry gives its
+ * single-output twin's results bit for bit.
+ * tgp_batch_multi_work_doubles: sum_b (N_b + r) * ld_b doubles (the outputs ride as rows N_b .. N_b + r - 1).
+ * tgp_loglike_batch_multi: out = {sum_c logL_c, sum_c chi2_c, logdet} per problem.  want_alpha == 0: out, info, the
+ *   factor and the rows L^-1 Y equal tgp_loglike_multi (row_end == NULL) on that problem alone bit for bit, alpha =
+ *   L^-1 Y.  want_alpha != 0: each column of alpha = K^-1 Y equals tgp_loglike_batch(want_alpha != 0) on that column
+ *   alone bit for bit.
+ * tgp_loglike_grad_batch_multi: out in the TGP_GRAD_BATCH_OUT layout with the joint logL and its gradient
+ *   (w_ij = sum_c alpha_ic alpha_jc - r Z_ij), scratch as tgp_loglike_grad_batch; agrees with tgp_loglike_grad_multi
+ *   to the rounding of alpha.
+ * tgp_predict_mean_batch_multi: equal bit for bit to tgp_predict_mean_multi wherever that call runs unsplit.
+ * tgp_loo_batch_multi: loo_mean_ic = y_ic - alpha_ic / Z_ii, loo_var_i = 1 / Z_ii - yerr2_i (sum N_b,). */
+int64_t tgp_batch_multi_work_doubles(const int64_t* off /*host*/, int32_t B, int32_t r);
+int tgp_loglike_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2,
+                            const int64_t* off /*host*/, int32_t B, const tgp_kernel_sum* ks /*host*/, double* work,
+                            double* alpha, int want_alpha, double* out, int32_t* info, void* stream);
+int tgp_loglike_grad_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2,
+                                 const int64_t* off /*host*/, int32_t B, const tgp_kernel_sum* ks /*host*/,
+                                 double* work, double* alpha, double* out, int32_t* info, double* scratch,
+                                 void* stream);
+int tgp_predict_mean_batch_multi(const double* Xs, const int64_t* soff /*host*/, const double* X,
+                                 const int64_t* off /*host*/, int32_t B, const tgp_kernel_sum* ks /*host*/,
+                                 const double* alpha, int32_t r, double* mean, void* stream);
+int tgp_loo_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2, const int64_t* off /*host*/,
+                        int32_t B, const tgp_kernel_sum* ks /*host*/, double* work, double* alpha, double* scratch,
+                        double* loo_mean, double* loo_var, int32_t* info, void* stream);
 
 /* ---- (4) predict ----------------------------------------------------------------------------- */
 

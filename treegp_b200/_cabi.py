@@ -85,6 +85,11 @@ SIGNATURES = {
     "tgp_predict_var_batch_work_doubles": [_vp, _vp, _i32, _i64],
     "tgp_predict_var_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp],
     "tgp_loo_batch": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tgp_batch_multi_work_doubles": [_vp, _i32, _i32],
+    "tgp_loglike_batch_multi": [_vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, ctypes.c_int, _vp, _vp, _vp],
+    "tgp_loglike_grad_batch_multi": [_vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
+    "tgp_predict_mean_batch_multi": [_vp, _vp, _vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp],
+    "tgp_loo_batch_multi": [_vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "tgp_predict_var_env": [_vp, _i64, _vp, _i64, _kp, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp],
     "tgp_predict_mean": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp],
     "tgp_predict_mean_trunc": [_vp, _i64, _vp, _i64, _kp, _vp, _vp, _vp, _vp],
@@ -122,6 +127,7 @@ _RESTYPES = {"tgp_last_error": ctypes.c_char_p, "tgp_pairbin_work_doubles": ctyp
              "tgp_selinv_work_doubles": ctypes.c_int64, "tgp_loglike_grad_sum_work_doubles": ctypes.c_int64,
              "tgp_loglike_grad_multi_work_doubles": ctypes.c_int64,
              "tgp_predict_work_doubles": ctypes.c_int64, "tgp_batch_work_doubles": ctypes.c_int64,
+             "tgp_batch_multi_work_doubles": ctypes.c_int64,
              "tgp_loglike_grad_batch_work_doubles": ctypes.c_int64, "tgp_predict_var_batch_work_doubles": ctypes.c_int64,
              "tgp_bootbin_work_bytes": ctypes.c_int64, "tgp_bootbin_sums_doubles": ctypes.c_int64, "tgp_profile_qcut": ctypes.c_double}
 

@@ -333,10 +333,11 @@ def batch_offsets(sizes):
     return np.ascontiguousarray(np.concatenate([[0], np.cumsum(np.asarray(sizes, dtype=np.int64))]), dtype=np.int64)
 
 
-def batch_work_doubles(sizes):
-    """Workspace of tgp_loglike_batch: sum_b (N_b + 1) * ld_b doubles, ld_b = N_b rounded up to even."""
+def batch_work_doubles(sizes, r=1):
+    """Workspace of tgp_loglike_batch_multi with r outputs: sum_b (N_b + r) * ld_b doubles, ld_b = N_b rounded up to
+    even."""
     n = np.asarray(sizes, dtype=np.int64)
-    return int(np.sum((n + 1) * ((n + 1) & ~1)))
+    return int(np.sum((n + r) * ((n + 1) & ~1)))
 
 
 def grad_batch_scratch_doubles(sizes):
@@ -352,13 +353,14 @@ def grad_batch_scratch_doubles(sizes):
     return int(np.sum(np.maximum(selinv, partials) + ((nblk + 1) & ~1)))
 
 
-def plan_batch_chunks(sizes, budget_bytes, scratch=False):
-    """Split problems with `sizes` points, in order, into consecutive chunks whose loglike_batch workspace (plus, with
-    scratch=True, the loglike_grad_batch scratch) fits `budget_bytes`; a problem larger than the budget gets a chunk of
-    its own.  Pure host function: returns a list of (start, stop) index pairs covering range(len(sizes))."""
+def plan_batch_chunks(sizes, budget_bytes, scratch=False, r=1):
+    """Split problems with `sizes` points, in order, into consecutive chunks whose loglike_batch workspace for r
+    outputs (plus, with scratch=True, the loglike_grad_batch scratch) fits `budget_bytes`; a problem larger than the
+    budget gets a chunk of its own.  Pure host function: returns a list of (start, stop) index pairs covering
+    range(len(sizes))."""
     chunks, start, used = [], 0, 0
     for b, n in enumerate(sizes):
-        need = 8 * batch_work_doubles([n]) + (8 * grad_batch_scratch_doubles([n]) if scratch else 0)
+        need = 8 * batch_work_doubles([n], r) + (8 * grad_batch_scratch_doubles([n]) if scratch else 0)
         if b > start and used + need > budget_bytes:
             chunks.append((start, b))
             start, used = b, 0
@@ -385,72 +387,82 @@ def _check_batch_inputs(X, sizes, descs):
 
 
 def loglike_batch(X, y, yerr2, sizes, descs, want_alpha=False, budget_bytes=4 << 30):
-    """tgp_loglike_batch over B problems: X (sum N_b, ndim), y and yerr2 (sum N_b,) concatenated device tensors,
-    problem b owning `sizes[b]` consecutive rows; descs: B descriptors (TgpKernel or TgpKernelSum).  The problems are
-    put through in chunks whose workspace fits `budget_bytes` (plan_batch_chunks); the results do not depend on the
-    chunking.  Returns (out (B, 3) = logL, chi2, logdet per problem; info (B,); alpha (sum N_b,): K^-1 y with
-    want_alpha, else L^-1 y)."""
+    """tgp_loglike_batch_multi over B problems: X (sum N_b, ndim), y (sum N_b,) or (sum N_b, r) for r outputs sharing
+    each problem's kernel, and yerr2 (sum N_b,) concatenated device tensors, problem b owning `sizes[b]` consecutive
+    rows; descs: B descriptors (TgpKernel or TgpKernelSum).  The problems are put through in chunks whose workspace
+    fits `budget_bytes` (plan_batch_chunks); the results do not depend on the chunking.  Returns (out (B, 3) = logL,
+    chi2, logdet per problem, joint over the outputs; info (B,); alpha, shaped as y: K^-1 y with want_alpha, else
+    L^-1 y)."""
     X = as_points(X)
     sizes = [int(n) for n in sizes]
     _check_batch_inputs(X, sizes, descs)
+    r = _outputs(y, X.shape[0], "y")
+    y = y.contiguous()
     off = batch_offsets(sizes)
     B = len(sizes)
     out = torch.empty((B, 3), dtype=F64, device=X.device)
     info = torch.empty(B, dtype=torch.int32, device=X.device)
-    alpha = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    alpha = torch.empty(y.shape, dtype=F64, device=X.device)
     lib = _cabi.load()
-    for b0, b1 in plan_batch_chunks(sizes, budget_bytes):
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, r=r):
         r0, r1 = int(off[b0]), int(off[b1])
         o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
-        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        work = torch.empty(batch_work_doubles(sizes[b0:b1], r), dtype=F64, device=X.device)
         ks = _ksum_array(descs[b0:b1])
-        check(lib.tgp_loglike_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
-                                    ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]), int(bool(want_alpha)),
-                                    _p(out[b0:b1]), _p(info[b0:b1]), _stream()), "tgp_loglike_batch")
+        check(lib.tgp_loglike_batch_multi(_p(X[r0:r1]), _p(y[r0:r1]), r, _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                          ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]),
+                                          int(bool(want_alpha)), _p(out[b0:b1]), _p(info[b0:b1]), _stream()),
+              "tgp_loglike_batch_multi")
     return out, info, alpha
 
 
 def loglike_grad_batch(X, y, yerr2, sizes, descs, budget_bytes=4 << 30):
-    """tgp_loglike_grad_batch over B problems, arguments as loglike_batch: each problem's log-likelihood and its
-    gradient in one pass, in chunks whose workspace plus scratch fit `budget_bytes` (plan_batch_chunks(scratch=True));
-    the results do not depend on the chunking.  Returns (out (B, TGP_GRAD_BATCH_OUT): per problem the layout of
-    loglike_grad for a sum, {logL, chi2, logdet, 4 derivatives per term, d / d ln white}, zero-padded; info (B,);
-    alpha (sum N_b,) = K^-1 y)."""
+    """tgp_loglike_grad_batch_multi over B problems, arguments as loglike_batch: each problem's (joint) log-likelihood
+    and its gradient in one pass, in chunks whose workspace plus scratch fit `budget_bytes`
+    (plan_batch_chunks(scratch=True)); the results do not depend on the chunking.  Returns (out (B,
+    TGP_GRAD_BATCH_OUT): per problem the layout of loglike_grad for a sum, {logL, chi2, logdet, 4 derivatives per term,
+    d / d ln white}, zero-padded; info (B,); alpha = K^-1 y, shaped as y)."""
     X = as_points(X)
     sizes = [int(n) for n in sizes]
     _check_batch_inputs(X, sizes, descs)
+    r = _outputs(y, X.shape[0], "y")
+    y = y.contiguous()
     off = batch_offsets(sizes)
     B = len(sizes)
     out = torch.empty((B, _cabi.GRAD_BATCH_OUT), dtype=F64, device=X.device)
     info = torch.empty(B, dtype=torch.int32, device=X.device)
-    alpha = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    alpha = torch.empty(y.shape, dtype=F64, device=X.device)
     lib = _cabi.load()
-    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True):
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True, r=r):
         r0, r1 = int(off[b0]), int(off[b1])
         o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
-        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        work = torch.empty(batch_work_doubles(sizes[b0:b1], r), dtype=F64, device=X.device)
         scratch = torch.empty(grad_batch_scratch_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
         ks = _ksum_array(descs[b0:b1])
-        check(lib.tgp_loglike_grad_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
-                                         ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]), _p(out[b0:b1]),
-                                         _p(info[b0:b1]), _p(scratch), _stream()), "tgp_loglike_grad_batch")
+        check(lib.tgp_loglike_grad_batch_multi(_p(X[r0:r1]), _p(y[r0:r1]), r, _p(yerr2[r0:r1]), _host_i64(o),
+                                               b1 - b0, ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha[r0:r1]),
+                                               _p(out[b0:b1]), _p(info[b0:b1]), _p(scratch), _stream()),
+              "tgp_loglike_grad_batch_multi")
     return out, info, alpha
 
 
 def predict_mean_batch(Xs, ssizes, X, sizes, descs, alpha):
-    """tgp_predict_mean_batch: mean rows of problem b = K_b(Xs_b, X_b) alpha_b (the full sum), with Xs (sum M_b, ndim)
-    and X, alpha concatenated as for loglike_batch.  Returns the (sum M_b,) device tensor of means."""
+    """tgp_predict_mean_batch_multi: mean rows of problem b = K_b(Xs_b, X_b) alpha_b (the full sum), with Xs
+    (sum M_b, ndim) and X, alpha ((sum N_b,) or (sum N_b, r)) concatenated as for loglike_batch.  Returns the device
+    tensor of means, (sum M_b,) or (sum M_b, r) as alpha."""
     Xs, X = as_points(Xs), as_points(X)
     sizes, ssizes = [int(n) for n in sizes], [int(m) for m in ssizes]
     _check_batch_inputs(X, sizes, descs)
     if len(ssizes) != len(sizes) or Xs.shape[0] != int(np.sum(ssizes)):
         raise ValueError("need one test-point count per problem, adding up to the rows of Xs")
     _check_dims(descs[0], X, Xs)
-    mean = torch.empty(Xs.shape[0], dtype=F64, device=X.device)
+    r = _outputs(alpha, X.shape[0], "alpha")
+    alpha = alpha.contiguous()
+    mean = torch.empty((Xs.shape[0],) + tuple(alpha.shape[1:]), dtype=F64, device=X.device)
     soff, off, ks = batch_offsets(ssizes), batch_offsets(sizes), _ksum_array(descs)   # alive during the call
-    check(_cabi.load().tgp_predict_mean_batch(_p(Xs), _host_i64(soff), _p(X), _host_i64(off), len(sizes),
-                                              ctypes.cast(ks, ctypes.c_void_p), _p(alpha), _p(mean), _stream()),
-          "tgp_predict_mean_batch")
+    check(_cabi.load().tgp_predict_mean_batch_multi(_p(Xs), _host_i64(soff), _p(X), _host_i64(off), len(sizes),
+                                                    ctypes.cast(ks, ctypes.c_void_p), _p(alpha), r, _p(mean),
+                                                    _stream()), "tgp_predict_mean_batch_multi")
     return mean
 
 
@@ -518,29 +530,32 @@ def predict_var_batch(Xs, ssizes, X, y, yerr2, sizes, descs, budget_bytes=4 << 3
 
 
 def loo_batch(X, y, yerr2, sizes, descs, budget_bytes=4 << 30):
-    """Leave-one-out predictions of every problem (tgp_loo_batch), arguments as loglike_batch, in chunks whose
-    workspace plus scratch fit `budget_bytes` (plan_batch_chunks(scratch=True)): mean_i = y_i - alpha_i / Z_ii and
-    var_i = 1 / Z_ii - yerr2_i in residual space, Z = K^-1.  Returns (mean, var, info): (sum N_b,), (sum N_b,), (B,);
+    """Leave-one-out predictions of every problem (tgp_loo_batch_multi), arguments as loglike_batch, in chunks whose
+    workspace plus scratch fit `budget_bytes` (plan_batch_chunks(scratch=True)): mean_ic = y_ic - alpha_ic / Z_ii and
+    var_i = 1 / Z_ii - yerr2_i in residual space, Z = K^-1.  Returns (mean, shaped as y; var (sum N_b,); info (B,));
     the rows of a problem with info != 0 are NaN."""
     X = as_points(X)
     sizes = [int(n) for n in sizes]
     _check_batch_inputs(X, sizes, descs)
+    r = _outputs(y, X.shape[0], "y")
+    y = y.contiguous()
     off = batch_offsets(sizes)
     B = len(sizes)
-    mean = torch.empty(int(off[-1]), dtype=F64, device=X.device)
+    mean = torch.empty(y.shape, dtype=F64, device=X.device)
     var = torch.empty(int(off[-1]), dtype=F64, device=X.device)
     info = torch.empty(B, dtype=torch.int32, device=X.device)
     lib = _cabi.load()
-    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True):
+    for b0, b1 in plan_batch_chunks(sizes, budget_bytes, scratch=True, r=r):
         r0, r1 = int(off[b0]), int(off[b1])
         o = np.ascontiguousarray(off[b0:b1 + 1] - off[b0])
-        work = torch.empty(batch_work_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
+        work = torch.empty(batch_work_doubles(sizes[b0:b1], r), dtype=F64, device=X.device)
         scratch = torch.empty(grad_batch_scratch_doubles(sizes[b0:b1]), dtype=F64, device=X.device)
-        alpha = torch.empty(r1 - r0, dtype=F64, device=X.device)
+        alpha = torch.empty(y[r0:r1].shape, dtype=F64, device=X.device)
         ks = _ksum_array(descs[b0:b1])
-        check(lib.tgp_loo_batch(_p(X[r0:r1]), _p(y[r0:r1]), _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
-                                ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha), _p(scratch), _p(mean[r0:r1]),
-                                _p(var[r0:r1]), _p(info[b0:b1]), _stream()), "tgp_loo_batch")
+        check(lib.tgp_loo_batch_multi(_p(X[r0:r1]), _p(y[r0:r1]), r, _p(yerr2[r0:r1]), _host_i64(o), b1 - b0,
+                                      ctypes.cast(ks, ctypes.c_void_p), _p(work), _p(alpha), _p(scratch),
+                                      _p(mean[r0:r1]), _p(var[r0:r1]), _p(info[b0:b1]), _stream()),
+              "tgp_loo_batch_multi")
     return mean, var, info
 
 

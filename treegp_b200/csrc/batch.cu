@@ -1,6 +1,8 @@
 // Batches of independent small problems: B likelihood evaluations (tgp_loglike_batch), B likelihoods with their
 // gradients (tgp_loglike_grad_batch), B posterior means (tgp_predict_mean_batch), B diagonal predictive variances
-// (tgp_predict_var_batch) or B sets of leave-one-out predictions (tgp_loo_batch) per call.
+// (tgp_predict_var_batch) or B sets of leave-one-out predictions (tgp_loo_batch) per call.  The _multi entries take r
+// outputs per problem sharing its kernel, as tgp_loglike_multi does for one problem: they ride through the
+// factorisation as r extra rows, and every later step reads them as an N x r row-major block.
 //
 // A problem of a few hundred to a few thousand points leaves the B200 idle: its factorisation is a chain of small
 // launches (8 panel launches and one update per 512 columns, at most ~70 CTAs each), so its time is launch latency.
@@ -8,9 +10,11 @@
 // problem, each CTA picks its problem from blockIdx.x and runs the body of the single-problem kernel on that
 // problem's slice (kmat.cu, dense.cu, predict.cu), and CTAs of problems without work at that step exit.  So a
 // problem's K, factor, logL and info are what tgp_loglike_sum (dense) gives on it alone, bit for bit, whatever else
-// shares the batch.  The only new arithmetic is the backward sweep of want_alpha (one CTA per problem, below).  The
-// gradient adds the selected inverse, contraction and finish of tgp_loglike_grad_sum in the same form (selinv.cu).
+// shares the batch.  The only new arithmetic is the backward sweep of want_alpha (one CTA per problem and group of
+// outputs, below).  The gradient adds the selected inverse, contraction and finish of tgp_loglike_grad_sum in the
+// same form (selinv.cu).
 #include <string.h>
+#include <algorithm>
 #include <vector>
 #include "tgp_common.cuh"
 #include "profile_policy.cuh"
@@ -58,8 +62,13 @@ static int check_batch(const char* fn, const int64_t* off, int32_t B, const tgp_
   return TGP_OK;
 }
 
-extern "C" int64_t tgp_batch_work_doubles(const int64_t* off, int32_t B) {
-  const char* fn = __func__;
+static int check_outputs(const char* fn, int32_t r) {
+  BATCH_CHECK(r >= 1 && r <= TGP_MAX_RHS, "number of outputs r must be 1 .. TGP_MAX_RHS");
+  return TGP_OK;
+}
+
+static int64_t work_doubles(const char* fn, const int64_t* off, int32_t B, int32_t r) {
+  if (check_outputs(fn, r)) return TGP_ERR_INVALID;
   if (B < 1) {
     tgp_set_error("%s: invalid argument: B must be >= 1", fn);
     return TGP_ERR_INVALID;
@@ -68,9 +77,15 @@ extern "C" int64_t tgp_batch_work_doubles(const int64_t* off, int32_t B) {
   int64_t total = 0;
   for (int32_t b = 0; b < B; ++b) {
     const int64_t n = off[b + 1] - off[b];
-    total += (n + 1) * even_ld(n);
+    total += (n + r) * even_ld(n);
   }
   return total;
+}
+
+extern "C" int64_t tgp_batch_work_doubles(const int64_t* off, int32_t B) { return work_doubles(__func__, off, B, 1); }
+
+extern "C" int64_t tgp_batch_multi_work_doubles(const int64_t* off, int32_t B, int32_t r) {
+  return work_doubles(__func__, off, B, r);
 }
 
 // The per-call device tables: problem descriptors, kernel descriptors, the problem lists of every profile class,
@@ -131,60 +146,82 @@ static int stage_tables(BatchTables& T, const std::vector<TgpBatchProb>& prob, c
   return TGP_OK;
 }
 
-// y into row N of every block (to_alpha == 0), or row N (= L^-1 y after the factorisation) into alpha.
+// Y (N x r, row-major) into rows N .. N + r - 1 of every block (to_alpha == 0), or those rows (= L^-1 y after the
+// factorisation) into alpha (N x r), as multi_transpose_kernel moves them for one problem.
 __global__ void __launch_bounds__(256)
 batch_yrow_kernel(const TgpBatchProb* __restrict__ pr, int to_alpha) {
   const TgpBatchProb& p = pr[blockIdx.x];
-  double* row = p.A + p.N * p.ld;
+  double* rows = p.A + p.N * p.ld;
+  const int64_t r = p.r;
   for (int64_t i = threadIdx.x; i < p.N; i += blockDim.x) {
-    if (to_alpha) p.alpha[i] = row[i];
-    else row[i] = p.y[i];
+    for (int64_t c = 0; c < r; ++c) {
+      if (to_alpha) p.alpha[i * r + c] = rows[c * p.ld + i];
+      else rows[c * p.ld + i] = p.y[i * r + c];
+    }
   }
 }
 
-// Backward sweep alpha <- L^-T alpha, one CTA per problem (the persistent cooperative sweeps of trsv.cu take one
-// problem per launch).  Blocks of 64 unknowns from the last: the four row groups of the CTA form
-// sum_{i >= j1} L[i, j0 + c] x_i for the block's 64 columns (each L entry is read once, rows coalesced), then warp 0
-// solves the 64 x 64 diagonal block by substitution with shuffles.  x lives in shared memory.
+// Backward sweep alpha <- L^-T alpha for G outputs of a problem per CTA (the persistent cooperative sweeps of trsv.cu
+// take one problem per launch); grid (problem, group of G outputs).  Blocks of 64 unknowns from the last: the four row
+// groups of the CTA form sum_{i >= j1} L[i, j0 + c] x_qi for the block's 64 columns and all G outputs q (each L entry
+// is read once per CTA, rows coalesced), then warp q solves the 64 x 64 diagonal block for output q by substitution
+// with shuffles.  Each output's arithmetic, and its order, is that of one output alone.  x lives in shared memory,
+// G columns of xp >= N doubles: G = 4 and N = 4096 take 128 KB.  The last group of r = 3, 5, 6, 7 has nq < G outputs;
+// its unused columns are zeroed, so that the shared sweep loop reads no uninitialised memory, and never written back.
 constexpr int BS_THREADS = 256;
 constexpr int BS_NB = 64;
-constexpr int BS_SMEM = (TGP_BATCH_MAX_N + BS_NB * (BS_NB + 1) + 4 * BS_NB) * 8;
+static size_t bs_smem(int G, int64_t xp) { return (size_t)(G * xp + BS_NB * (BS_NB + 1) + 4 * G * BS_NB) * 8; }
 
-__global__ void __launch_bounds__(BS_THREADS)
-backward_batch_kernel(const TgpBatchProb* __restrict__ pr) {
+template <int G>
+__global__ void __launch_bounds__(BS_THREADS, 2)
+backward_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t xp) {
   extern __shared__ double bsm[];
-  double* x = bsm;                                 // N unknowns
-  double* Ld = bsm + TGP_BATCH_MAX_N;              // diagonal block, pitch BS_NB + 1
-  double* part = Ld + BS_NB * (BS_NB + 1);         // 4 partial sums per column
+  double* x = bsm;                                 // G x xp unknowns
+  double* Ld = bsm + G * xp;                       // diagonal block, pitch BS_NB + 1
+  double* part = Ld + BS_NB * (BS_NB + 1);         // G x 4 partial sums per column
   const TgpBatchProb& p = pr[blockIdx.x];
-  const int64_t N = p.N, ld = p.ld;
+  const int N = (int)p.N, r = (int)p.r;            // N <= TGP_BATCH_MAX_N: int indices
+  const int64_t ld = p.ld;
+  const int q0 = (int)blockIdx.y * G;              // first output of this CTA
+  const int nq = r - q0 < G ? r - q0 : G;          // outputs of this CTA
   const double* L = p.A;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int c = tid & (BS_NB - 1), g = tid / BS_NB;
-  for (int64_t i = tid; i < N; i += BS_THREADS) x[i] = p.alpha[i];
+  for (int q = 0; q < G; ++q) {   // the columns of outputs beyond r (last group) are zeros, swept and never written
+    for (int i = tid; i < N; i += BS_THREADS) x[q * xp + i] = q < nq ? p.alpha[(int64_t)i * r + q0 + q] : 0.0;
+  }
   __syncthreads();
-  for (int64_t j0 = (N - 1) / BS_NB * BS_NB; j0 >= 0; j0 -= BS_NB) {
-    const int nb = (int)(N - j0 < BS_NB ? N - j0 : BS_NB);
-    const int64_t j1 = j0 + nb;
-    double s = 0.0;
+  for (int j0 = (N - 1) / BS_NB * BS_NB; j0 >= 0; j0 -= BS_NB) {
+    const int nb = N - j0 < BS_NB ? N - j0 : BS_NB;
+    const int j1 = j0 + nb;
+    double s[G];
+#pragma unroll
+    for (int q = 0; q < G; ++q) s[q] = 0.0;
     if (c < nb) {
 #pragma unroll 4
-      for (int64_t i = j1 + g; i < N; i += 4) s = fma(L[i * ld + j0 + c], x[i], s);
+      for (int i = j1 + g; i < N; i += 4) {
+        const double l = L[i * ld + j0 + c];
+#pragma unroll
+        for (int q = 0; q < G; ++q) s[q] = fma(l, x[q * xp + i], s[q]);
+      }
     }
-    part[g * BS_NB + c] = s;
+#pragma unroll
+    for (int q = 0; q < G; ++q) part[(4 * q + g) * BS_NB + c] = s[q];
     for (int idx = tid; idx < BS_NB * BS_NB; idx += BS_THREADS) {
-      const int r = idx / BS_NB, cc = idx % BS_NB;
-      Ld[r * (BS_NB + 1) + cc] = (r < nb && cc <= r) ? L[(j0 + r) * ld + j0 + cc] : 0.0;
+      const int rr = idx / BS_NB, cc = idx % BS_NB;
+      Ld[rr * (BS_NB + 1) + cc] = (rr < nb && cc <= rr) ? L[(j0 + rr) * ld + j0 + cc] : 0.0;
     }
     __syncthreads();
-    if (warp == 0) {
-      // lane owns unknowns j0 + lane (r0) and j0 + 32 + lane (r1)
+    if (warp < nq) {
+      // lane owns unknowns j0 + lane (r0) and j0 + 32 + lane (r1) of output `warp`
+      double* xq = x + warp * xp;
+      const double* pq = part + 4 * warp * BS_NB;
       double r0 = 0.0, r1 = 0.0;
       if (lane < nb)
-        r0 = x[j0 + lane] - (((part[lane] + part[BS_NB + lane]) + part[2 * BS_NB + lane]) + part[3 * BS_NB + lane]);
+        r0 = xq[j0 + lane] - (((pq[lane] + pq[BS_NB + lane]) + pq[2 * BS_NB + lane]) + pq[3 * BS_NB + lane]);
       if (lane + 32 < nb) {
         const int l = lane + 32;
-        r1 = x[j0 + l] - (((part[l] + part[BS_NB + l]) + part[2 * BS_NB + l]) + part[3 * BS_NB + l]);
+        r1 = xq[j0 + l] - (((pq[l] + pq[BS_NB + l]) + pq[2 * BS_NB + l]) + pq[3 * BS_NB + l]);
       }
       for (int i = nb - 1; i >= 0; --i) {
         const double xi = __shfl_sync(0xffffffffu, i < 32 ? r0 : r1, i & 31) / Ld[i * (BS_NB + 1) + i];
@@ -195,38 +232,59 @@ backward_batch_kernel(const TgpBatchProb* __restrict__ pr) {
         if (lane < i) r0 = fma(-Ld[i * (BS_NB + 1) + lane], xi, r0);
         if (lane + 32 < i) r1 = fma(-Ld[i * (BS_NB + 1) + lane + 32], xi, r1);
       }
-      if (lane < nb) x[j0 + lane] = r0;
-      if (lane + 32 < nb) x[j0 + lane + 32] = r1;
+      if (lane < nb) xq[j0 + lane] = r0;
+      if (lane + 32 < nb) xq[j0 + lane + 32] = r1;
     }
     __syncthreads();
   }
-  for (int64_t i = tid; i < N; i += BS_THREADS) p.alpha[i] = x[i];
+  for (int q = 0; q < nq; ++q) {
+    for (int i = tid; i < N; i += BS_THREADS) p.alpha[(int64_t)i * r + q0 + q] = x[q * xp + i];
+  }
 }
 
-// The chain of tgp_loglike_batch on checked arguments, with the tables staged into T (plus `extra` bytes) and their
-// host copy in prob.  out: 3 B doubles, or nullptr for T.extra's first 3 B doubles.
-static int loglike_batch_run(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
-                             const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
-                             int32_t* info, cudaStream_t st, BatchTables& T, std::vector<TgpBatchProb>& prob,
-                             const std::vector<unsigned char>& extra) {
+// Outputs per CTA of the backward sweep: one CTA reads the factor for up to 4 outputs (x of 4 outputs at N = 4096
+// fills 128 KB of shared memory; 8 would not fit).
+static int backward_group(int64_t r) { return r == 1 ? 1 : (r == 2 ? 2 : 4); }
+
+template <int G>
+static int backward_batch_launch(const TgpBatchProb* pr, int32_t B, int64_t r, int64_t max_n, cudaStream_t st) {
+  static TgpPerDeviceOnce attr_once;
+  if (tgp_first_use_on_device(attr_once))
+    TGP_CUDA(cudaFuncSetAttribute(backward_batch_kernel<G>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)bs_smem(G, TGP_BATCH_MAX_N)));
+  const int64_t xp = even_ld(max_n);
+  backward_batch_kernel<G><<<dim3((unsigned)B, (unsigned)tgp_cdiv(r, (int64_t)G)), BS_THREADS, bs_smem(G, xp), st>>>(
+      pr, xp);
+  TGP_LAUNCH_CHECK();
+  return TGP_OK;
+}
+
+// The chain of tgp_loglike_batch (r outputs per problem) on checked arguments, with the tables staged into T (plus
+// `extra` bytes) and their host copy in prob.  out: 3 B doubles, or nullptr for T.extra's first 3 B doubles.
+static int loglike_batch_run(const double* X, const double* y, int32_t r, const double* yerr2, const int64_t* off,
+                             int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha,
+                             double* out, int32_t* info, cudaStream_t st, BatchTables& T,
+                             std::vector<TgpBatchProb>& prob, const std::vector<unsigned char>& extra) {
   int rc;
   const int ndim = ks[0].ndim;
   prob.assign(B, TgpBatchProb{});
   std::vector<int> cls(B);
   std::vector<int64_t> Nh(B);
-  int64_t woff = 0;
+  int64_t woff = 0, max_n = 0;
   for (int32_t b = 0; b < B; ++b) {
     const int64_t r0 = off[b], n = off[b + 1] - off[b];
     TgpBatchProb& p = prob[b];
     p = TgpBatchProb{};
     p.X = X + r0 * ndim;
-    p.y = y + r0;
+    p.y = y + r0 * r;
     p.yerr2 = yerr2 + r0;
     p.A = work + woff;
-    p.alpha = alpha + r0;
+    p.alpha = alpha + r0 * r;
     p.N = Nh[b] = n;
     p.ld = even_ld(n);
-    woff += (n + 1) * p.ld;
+    p.r = r;
+    woff += (n + r) * p.ld;
+    max_n = std::max(max_n, n);
     // the K build of tgp_kmat_sym_sum: the single-term kernel for one term without a white level
     cls[b] = (ks[b].nterms == 1 && ks[b].white == 0.0) ? ks[b].term[0].family : TGP_BATCH_SUM;
   }
@@ -240,32 +298,46 @@ static int loglike_batch_run(const double* X, const double* y, const double* yer
   }
   batch_yrow_kernel<<<(unsigned)B, 256, 0, st>>>(T.pr, 0);
   TGP_LAUNCH_CHECK();
-  rc = tgp_batch_potrf_rows(T.pr, Nh.data(), B, info, T.flags, st);
+  rc = tgp_batch_potrf_rows(T.pr, Nh.data(), B, r, info, T.flags, st);
   if (rc) return rc;
   batch_yrow_kernel<<<(unsigned)B, 256, 0, st>>>(T.pr, 1);
   TGP_LAUNCH_CHECK();
   if (want_alpha) {
-    static TgpPerDeviceOnce attr_once;
-    if (tgp_first_use_on_device(attr_once))
-      TGP_CUDA(cudaFuncSetAttribute(backward_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BS_SMEM));
-    backward_batch_kernel<<<(unsigned)B, BS_THREADS, BS_SMEM, st>>>(T.pr);
-    TGP_LAUNCH_CHECK();
+    switch (backward_group(r)) {
+      case 1: rc = backward_batch_launch<1>(T.pr, B, r, max_n, st); break;
+      case 2: rc = backward_batch_launch<2>(T.pr, B, r, max_n, st); break;
+      default: rc = backward_batch_launch<4>(T.pr, B, r, max_n, st); break;
+    }
+    if (rc) return rc;
   }
-  return tgp_batch_loglike_finish(T.pr, B, want_alpha, info, out, st);
+  return tgp_batch_loglike_finish(T.pr, B, r, want_alpha, info, out, st);
 }
 
-extern "C" int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
-                                 const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
-                                 int32_t* info, void* stream) {
-  const char* fn = __func__;
-  int rc = check_batch(fn, off, B, ks);
+static int loglike_batch_entry(const char* fn, const double* X, const double* y, int32_t r, const double* yerr2,
+                               const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha,
+                               int want_alpha, double* out, int32_t* info, void* stream) {
+  int rc = check_outputs(fn, r);
+  if (rc) return rc;
+  rc = check_batch(fn, off, B, ks);
   if (rc) return rc;
   BATCH_CHECK(X && y && yerr2 && work && alpha && out && info, "null pointer (X, y, yerr2, work, alpha, out, info)");
   BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
   BatchTables T;
   std::vector<TgpBatchProb> prob;
-  return loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, want_alpha, out, info, (cudaStream_t)stream, T, prob,
-                           std::vector<unsigned char>());
+  return loglike_batch_run(X, y, r, yerr2, off, B, ks, work, alpha, want_alpha, out, info, (cudaStream_t)stream, T,
+                           prob, std::vector<unsigned char>());
+}
+
+extern "C" int tgp_loglike_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                                 const tgp_kernel_sum* ks, double* work, double* alpha, int want_alpha, double* out,
+                                 int32_t* info, void* stream) {
+  return loglike_batch_entry(__func__, X, y, 1, yerr2, off, B, ks, work, alpha, want_alpha, out, info, stream);
+}
+
+extern "C" int tgp_loglike_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2,
+                                       const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work,
+                                       double* alpha, int want_alpha, double* out, int32_t* info, void* stream) {
+  return loglike_batch_entry(__func__, X, Y, r, yerr2, off, B, ks, work, alpha, want_alpha, out, info, stream);
 }
 
 extern "C" int64_t tgp_loglike_grad_sum_work_doubles(int64_t N, int32_t nterms);
@@ -284,12 +356,26 @@ extern "C" int64_t tgp_loglike_grad_batch_work_doubles(const int64_t* off, int32
   return total;
 }
 
+// The arguments of tgp_loglike_grad_batch and tgp_loo_batch (and their _multi forms), in the order and with the
+// messages of the single-output entries: `nonnull` is the caller's null-pointer test, `null_msg` its message.
+static int check_selinv_batch(const char* fn, int32_t r, const int64_t* off, int32_t B, const tgp_kernel_sum* ks,
+                              bool nonnull, const char* null_msg, const double* work, const double* scratch) {
+  int rc = check_outputs(fn, r);
+  if (rc) return rc;
+  rc = check_batch(fn, off, B, ks);
+  if (rc) return rc;
+  BATCH_CHECK(nonnull, null_msg);
+  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
+  BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
+  return TGP_OK;
+}
+
 // tgp_loglike_batch(want_alpha = 1) and the batched selected inverse on checked arguments.  T.extra holds
 // {logL, chi2, logdet} per problem, then the scratch block of every problem (*scr on the device), then `tail`.
-static int selinv_batch_run(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
-                            const tgp_kernel_sum* ks, double* work, double* alpha, int32_t* info, double* scratch,
-                            cudaStream_t st, BatchTables& T, std::vector<TgpBatchProb>& prob, double* const** scr,
-                            const std::vector<unsigned char>& tail = std::vector<unsigned char>()) {
+static int selinv_batch_run(const double* X, const double* y, int32_t r, const double* yerr2, const int64_t* off,
+                            int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, int32_t* info,
+                            double* scratch, cudaStream_t st, BatchTables& T, std::vector<TgpBatchProb>& prob,
+                            double* const** scr, const std::vector<unsigned char>& tail = std::vector<unsigned char>()) {
   const size_t o_scr = align16((size_t)B * 3 * sizeof(double));
   const size_t o_tail = align16(o_scr + (size_t)B * sizeof(double*));
   std::vector<unsigned char> extra(o_tail + tail.size(), 0);
@@ -300,27 +386,23 @@ static int selinv_batch_run(const double* X, const double* y, const double* yerr
     scr_h[b] = scratch + soff;
     soff += tgp_loglike_grad_sum_work_doubles(off[b + 1] - off[b], TGP_MAX_TERMS);
   }
-  int rc = loglike_batch_run(X, y, yerr2, off, B, ks, work, alpha, 1, nullptr, info, st, T, prob, extra);
+  int rc = loglike_batch_run(X, y, r, yerr2, off, B, ks, work, alpha, 1, nullptr, info, st, T, prob, extra);
   if (rc) return rc;
   *scr = reinterpret_cast<double* const*>(T.extra + o_scr);
   return tgp_batch_selinv(T.pr, *scr, prob.data(), scr_h, B, st);
 }
 
-extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off,
-                                      int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, double* out,
-                                      int32_t* info, double* scratch, void* stream) {
-  const char* fn = __func__;
-  int rc = check_batch(fn, off, B, ks);
+static int loglike_grad_batch_entry(const char* fn, const double* X, const double* y, int32_t r, const double* yerr2,
+                                    const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work,
+                                    double* alpha, double* out, int32_t* info, double* scratch, void* stream) {
+  int rc = check_selinv_batch(fn, r, off, B, ks, X && y && yerr2 && work && alpha && out && info && scratch,
+                              "null pointer (X, y, yerr2, work, alpha, out, info, scratch)", work, scratch);
   if (rc) return rc;
-  BATCH_CHECK(X && y && yerr2 && work && alpha && out && info && scratch,
-              "null pointer (X, y, yerr2, work, alpha, out, info, scratch)");
-  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
-  BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   BatchTables T;
   std::vector<TgpBatchProb> prob;
   double* const* scr = nullptr;
-  rc = selinv_batch_run(X, y, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr);
+  rc = selinv_batch_run(X, y, r, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr);
   if (rc) return rc;
   const double* ll = reinterpret_cast<const double*>(T.extra);
   for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
@@ -330,17 +412,31 @@ extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const do
       for (int32_t b = 0; b < B; ++b) max_terms = ks[b].nterms > max_terms ? ks[b].nterms : max_terms;
     }
     rc = tgp_batch_grad_contract(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, scr, T.max_n[c],
-                                 max_terms, st);
+                                 max_terms, r, st);
     if (rc) return rc;
   }
   return tgp_batch_grad_finish(T.pr, T.kd, scr, B, info, ll, out, st);
 }
 
-extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, const double* X, const int64_t* off,
-                                      int32_t B, const tgp_kernel_sum* ks, const double* alpha, double* mean,
-                                      void* stream) {
-  const char* fn = __func__;
-  int rc = check_batch(fn, off, B, ks);
+extern "C" int tgp_loglike_grad_batch(const double* X, const double* y, const double* yerr2, const int64_t* off,
+                                      int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha, double* out,
+                                      int32_t* info, double* scratch, void* stream) {
+  return loglike_grad_batch_entry(__func__, X, y, 1, yerr2, off, B, ks, work, alpha, out, info, scratch, stream);
+}
+
+extern "C" int tgp_loglike_grad_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2,
+                                            const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work,
+                                            double* alpha, double* out, int32_t* info, double* scratch,
+                                            void* stream) {
+  return loglike_grad_batch_entry(__func__, X, Y, r, yerr2, off, B, ks, work, alpha, out, info, scratch, stream);
+}
+
+static int predict_mean_batch_entry(const char* fn, const double* Xs, const int64_t* soff, const double* X,
+                                    const int64_t* off, int32_t B, const tgp_kernel_sum* ks, const double* alpha,
+                                    int32_t r, double* mean, void* stream) {
+  int rc = check_outputs(fn, r);
+  if (rc) return rc;
+  rc = check_batch(fn, off, B, ks);
   if (rc) return rc;
   rc = check_offsets(fn, "soff", soff, B, 0, INT64_MAX);
   if (rc) return rc;
@@ -354,12 +450,13 @@ extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, con
     TgpBatchProb& p = prob[b];
     p = TgpBatchProb{};
     p.X = X + off[b] * ndim;
-    p.alpha = const_cast<double*>(alpha) + off[b];
+    p.alpha = const_cast<double*>(alpha) + off[b] * r;
     p.N = off[b + 1] - off[b];
     p.Xs = Xs + soff[b] * ndim;
-    p.mean = mean + soff[b];
+    p.mean = mean + soff[b] * r;
     p.M = soff[b + 1] - soff[b];
-    // tgp_predict_mean_sum: the single-term kernel for any one-term sum (no white term in K(Xs, X))
+    p.r = r;
+    // tgp_predict_mean_sum / _multi: the single-term kernel for any one-term sum (no white term in K(Xs, X))
     cls[b] = ks[b].nterms == 1 ? ks[b].term[0].family : TGP_BATCH_SUM;
   }
   BatchTables T;
@@ -367,52 +464,75 @@ extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, con
   if (rc) return rc;
   for (int c = 0; c < TGP_BATCH_NCLASS; ++c) {
     if (T.start[c + 1] == T.start[c] || T.max_m[c] == 0) continue;
-    rc = tgp_batch_predict_mean(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, T.max_m[c], st);
+    rc = tgp_batch_predict_mean(T.pr, T.kd, T.list + T.start[c], T.start[c + 1] - T.start[c], c, T.max_m[c], r, st);
     if (rc) return rc;
   }
   return TGP_OK;
 }
 
+extern "C" int tgp_predict_mean_batch(const double* Xs, const int64_t* soff, const double* X, const int64_t* off,
+                                      int32_t B, const tgp_kernel_sum* ks, const double* alpha, double* mean,
+                                      void* stream) {
+  return predict_mean_batch_entry(__func__, Xs, soff, X, off, B, ks, alpha, 1, mean, stream);
+}
+
+extern "C" int tgp_predict_mean_batch_multi(const double* Xs, const int64_t* soff, const double* X,
+                                            const int64_t* off, int32_t B, const tgp_kernel_sum* ks,
+                                            const double* alpha, int32_t r, double* mean, void* stream) {
+  return predict_mean_batch_entry(__func__, Xs, soff, X, off, B, ks, alpha, r, mean, stream);
+}
+
 // ---- leave-one-out predictions (tgp_loo_batch) ---------------------------------------------------------------------
 // One CTA per problem, in residual space, with the operations of GPInterpolation.loo_predict in the same order:
-// mean_i = y_i - alpha_i / Z_ii, var_i = 1 / Z_ii - yerr2_i; NaN for a problem with info != 0.
+// mean_ic = y_ic - alpha_ic / Z_ii for each output c, var_i = 1 / Z_ii - yerr2_i once per point; NaN for a problem
+// with info != 0.
 __global__ void __launch_bounds__(256)
 loo_finish_batch_kernel(const TgpBatchProb* __restrict__ pr, const int64_t* __restrict__ off,
                         const int32_t* __restrict__ info, double* __restrict__ mean, double* __restrict__ var) {
   const TgpBatchProb& p = pr[blockIdx.x];
-  const int64_t r0 = off[blockIdx.x];
+  const int64_t r0 = off[blockIdx.x], r = p.r;
   const bool ok = info[blockIdx.x] == 0;
   const double nan = __longlong_as_double(0x7ff8000000000000ll);
   for (int64_t i = threadIdx.x; i < p.N; i += blockDim.x) {
     const double z = p.A[i * p.ld + i];
-    mean[r0 + i] = ok ? p.y[i] - p.alpha[i] / z : nan;
+    for (int64_t c = 0; c < r; ++c) mean[(r0 + i) * r + c] = ok ? p.y[i * r + c] - p.alpha[i * r + c] / z : nan;
     var[r0 + i] = ok ? 1.0 / z - p.yerr2[i] : nan;
   }
 }
 
-extern "C" int tgp_loo_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
-                             const tgp_kernel_sum* ks, double* work, double* alpha, double* scratch, double* loo_mean,
-                             double* loo_var, int32_t* info, void* stream) {
-  const char* fn = __func__;
-  int rc = check_batch(fn, off, B, ks);
+static int loo_batch_entry(const char* fn, const double* X, const double* y, int32_t r, const double* yerr2,
+                           const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work, double* alpha,
+                           double* scratch, double* loo_mean, double* loo_var, int32_t* info, void* stream) {
+  int rc = check_selinv_batch(fn, r, off, B, ks,
+                              X && y && yerr2 && work && alpha && scratch && loo_mean && loo_var && info,
+                              "null pointer (X, y, yerr2, work, alpha, scratch, loo_mean, loo_var, info)", work, scratch);
   if (rc) return rc;
-  BATCH_CHECK(X && y && yerr2 && work && alpha && scratch && loo_mean && loo_var && info,
-              "null pointer (X, y, yerr2, work, alpha, scratch, loo_mean, loo_var, info)");
-  BATCH_CHECK(((uintptr_t)work & 15) == 0, "work must be 16-byte aligned");
-  BATCH_CHECK(((uintptr_t)scratch & 15) == 0, "scratch must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   std::vector<unsigned char> tail((size_t)(B + 1) * sizeof(int64_t));   // the offsets, for the finish
   memcpy(tail.data(), off, tail.size());
   BatchTables T;
   std::vector<TgpBatchProb> prob;
   double* const* scr = nullptr;
-  rc = selinv_batch_run(X, y, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr, tail);
+  rc = selinv_batch_run(X, y, r, yerr2, off, B, ks, work, alpha, info, scratch, st, T, prob, &scr, tail);
   if (rc) return rc;
   const int64_t* off_d = reinterpret_cast<const int64_t*>(reinterpret_cast<const unsigned char*>(scr) +
                                                           align16((size_t)B * sizeof(double*)));
   loo_finish_batch_kernel<<<(unsigned)B, 256, 0, st>>>(T.pr, off_d, info, loo_mean, loo_var);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
+}
+
+extern "C" int tgp_loo_batch(const double* X, const double* y, const double* yerr2, const int64_t* off, int32_t B,
+                             const tgp_kernel_sum* ks, double* work, double* alpha, double* scratch, double* loo_mean,
+                             double* loo_var, int32_t* info, void* stream) {
+  return loo_batch_entry(__func__, X, y, 1, yerr2, off, B, ks, work, alpha, scratch, loo_mean, loo_var, info, stream);
+}
+
+extern "C" int tgp_loo_batch_multi(const double* X, const double* Y, int32_t r, const double* yerr2,
+                                   const int64_t* off, int32_t B, const tgp_kernel_sum* ks, double* work,
+                                   double* alpha, double* scratch, double* loo_mean, double* loo_var, int32_t* info,
+                                   void* stream) {
+  return loo_batch_entry(__func__, X, Y, r, yerr2, off, B, ks, work, alpha, scratch, loo_mean, loo_var, info, stream);
 }
 
 // ---- predictive variance (tgp_predict_var_batch) -------------------------------------------------------------------

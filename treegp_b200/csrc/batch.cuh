@@ -1,5 +1,5 @@
 // Batches of independent problems (tgp_loglike_batch, tgp_loglike_grad_batch, tgp_predict_mean_batch,
-// tgp_predict_var_batch, tgp_loo_batch): the per-problem
+// tgp_predict_var_batch, tgp_loo_batch and the _multi entries): the per-problem
 // table the batched kernels read, and the launchers that kmat.cu, dense.cu, selinv.cu and predict.cu provide to
 // batch.cu.  Every batched kernel
 // runs the body of its single-problem twin on one problem's slice, so each problem gets the single call's arithmetic.
@@ -10,13 +10,14 @@
 // One problem of a batch, as the device sees it (staged by batch.cu).
 struct TgpBatchProb {
   const double* X;       // N x ndim training points
-  const double* y;       // N values
+  const double* y;       // N x r values, row-major
   const double* yerr2;   // N diagonal additions
-  double* A;             // (N + 1) x ld block of the workspace: K, then L, with y riding along as row N
-  double* alpha;         // N: L^-1 y, or K^-1 y after the backward sweep
+  double* A;             // (N + r) x ld block of the workspace: K, then L, with output c riding along as row N + c
+  double* alpha;         // N x r: L^-1 y, or K^-1 y after the backward sweep
   const double* Xs;      // M x ndim test points (predict)
-  double* mean;          // M (predict)
+  double* mean;          // M x r (predict)
   int64_t N, M, ld;
+  int64_t r;             // outputs sharing the kernel, the same for every problem of a batch
 };
 
 // Profile class of a problem: its family (one term, and for the K build no white level), or a sum.  This is the
@@ -46,14 +47,16 @@ TGP_BATCH_FAMILY_PROFILE(TGP_FAM_MATERN52)
 // bound the sizes of those problems.  Nh: host copy of the problem sizes.
 int tgp_batch_kmat_sym(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
                        int64_t max_n, cudaStream_t st);
-// Cholesky of every problem's block with y riding along as row N (row N then holds L^-1 y); flags: B zeroed words.
-int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, int32_t* info, unsigned* flags,
-                         cudaStream_t st);
-// out[3 b ..] = {logL, chi2, logdet} from the factor and alpha, in the order of the single call's reductions.
-int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int want_alpha, const int32_t* info, double* out,
-                             cudaStream_t st);
+// Cholesky of every problem's block with its r outputs riding along as rows N .. N + r - 1 (which then hold
+// L^-1 y); flags: B zeroed words.
+int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, int64_t r, int32_t* info,
+                         unsigned* flags, cudaStream_t st);
+// out[3 b ..] = {logL, chi2, logdet} from the factor and alpha, in the order of the single call's reductions
+// (tgp_loglike_sum for r = 1, tgp_loglike_multi for r > 1).
+int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int64_t r, int want_alpha, const int32_t* info,
+                             double* out, cudaStream_t st);
 int tgp_batch_predict_mean(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
-                           int64_t max_m, cudaStream_t st);
+                           int64_t max_m, int r, cudaStream_t st);
 
 // ---- selected inverse of a batch (tgp_loglike_grad_batch) ----------------------------------------------------------
 // Step s of a problem with N points handles its block column nb - 1 - s (nb = ceil(N / TGP_OB)), as selinv_run does
@@ -154,7 +157,8 @@ int tgp_batch_var_rows(const TgpBatchProb* pr, const double* prior, int32_t B, i
 
 // The contraction of the problems `list` (profile class cls) into their scratch, then one finishing CTA per problem
 // writing out[b * TGP_GRAD_BATCH_OUT ..] from ll[3 b ..] = {logL, chi2, logdet}, the tile sums and info.
+// r > 1: the contraction of tgp_loglike_grad_multi, w_ij = sum_c alpha_ic alpha_jc - r Z_ij.
 int tgp_batch_grad_contract(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
-                            double* const* scr, int64_t max_n, int max_terms, cudaStream_t st);
+                            double* const* scr, int64_t max_n, int max_terms, int r, cudaStream_t st);
 int tgp_batch_grad_finish(const TgpBatchProb* pr, const KSumDesc* kd, double* const* scr, int32_t B,
                           const int32_t* info, const double* ll, double* out, cudaStream_t st);

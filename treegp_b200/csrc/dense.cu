@@ -1214,25 +1214,8 @@ __global__ void __launch_bounds__(1024)
 loglike_multi_finish_kernel(const double* __restrict__ L, int64_t N, int64_t ld, const double* __restrict__ Y, int r,
                             const double* __restrict__ W, int want_alpha, const int32_t* __restrict__ info,
                             double* __restrict__ out) {
-  __shared__ double s[32];
-  double a = 0.0;
-  for (int64_t i = threadIdx.x; i < N; i += blockDim.x) a += 2.0 * log(L[i * ld + i]);
-  const double logdet = block_sum_1024(a, s);
-  double chi2 = 0.0;
-  for (int c = 0; c < r; ++c) {
-    const double* w = W + c * ld;
-    double v = 0.0;
-    for (int64_t i = threadIdx.x; i < N; i += blockDim.x) v = want_alpha ? fma(Y[i * r + c], w[i], v) : fma(w[i], w[i], v);
-    chi2 += block_sum_1024(v, s);
-  }
-  if (threadIdx.x == 0) {
-    double ll = -0.5 * chi2 - 0.5 * (double)r * (double)N * log(2.0 * TGP_PI) - 0.5 * (double)r * logdet;
-    if (*info > 0 || isnan(ll)) ll = -INFINITY;   // as loglike_finish_kernel
-    if (*info < 0) ll = NAN;
-    out[0] = ll;
-    out[1] = chi2;
-    out[2] = logdet;
-  }
+  const int64_t wcol = ld, wrow = 1;   // output c in row c of W
+#include "multi_finish_body.cuh"
 }
 
 extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, const double* yerr2, int64_t N,
@@ -1274,8 +1257,8 @@ extern "C" int tgp_loglike_multi(const double* X, const double* Y, int32_t r, co
 }
 
 // ============================================================================================
-// Batches of independent problems (tgp_loglike_batch).  The schedule of potrf_blocked with y riding along as row N,
-// run once over the panel steps of the largest problem: every launch covers each problem that still has columns at
+// Batches of independent problems (tgp_loglike_batch).  The schedule of potrf_blocked with the r outputs riding along
+// as rows N .. N + r - 1, run once over the panel steps of the largest problem: every launch covers each problem that still has columns at
 // that step (CTAs of the others exit), and each CTA runs the body of the single-problem kernel on its problem's block.
 // For N >= 3 TGP_OB the single call takes the look-ahead driver, whose U1 / U2 updates split the same K = TGP_OB update
 // by columns: per element the same DMMA chain, so the factor is the same bit for bit.
@@ -1290,13 +1273,13 @@ panel_left_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int j, i
   const int w = (int)(N - k < TGP_OB ? N - k : TGP_OB);
   const int ndiag = (w + NB - 1) / NB;
   if (j >= ndiag) return;
-  const int64_t below = N - k - w + 1;
+  const int64_t below = N - k - w + pr[b].r;
   if ((int64_t)blockIdx.y >= (ndiag - j) + (below + NB - 1) / NB) return;
   const int64_t ld = pr[b].ld;
   panel_left_body(pr[b].A + k * ld + k, ld, w, below, j, info + b, k, flags + b, epoch, blockIdx.y);
 }
 
-// The trailing update of outer step k: C (rest + 1 x rest) -= L21 L21^T (lower), the y row included.
+// The trailing update of outer step k: C (rest + r x rest) -= L21 L21^T (lower), the output rows included.
 // grid: (problem, row tile * tiles_n + column tile).
 __global__ void __launch_bounds__(GEMM_THREADS, 2)
 gemm_trail_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int tiles_n) {
@@ -1305,14 +1288,15 @@ gemm_trail_batch_kernel(const TgpBatchProb* __restrict__ pr, int64_t k, int tile
   const int64_t w = N - k < TGP_OB ? N - k : TGP_OB, rest = N - k - w;
   if (rest <= 0) return;
   const int64_t m0 = (int64_t)(blockIdx.y / tiles_n) * BM, n0 = (int64_t)(blockIdx.y % tiles_n) * 64;
-  if (m0 >= rest + 1 || n0 >= rest) return;
+  const int64_t rows = rest + pr[b].r;
+  if (m0 >= rows || n0 >= rest) return;
   const int64_t ld = pr[b].ld;
   double* Ark = pr[b].A + (k + w) * ld + k;
-  gemm_nt_sub_tile<64, 4, 2>(Ark + w, rest + 1, rest, ld, Ark, ld, Ark, ld, w, 1, m0, n0);
+  gemm_nt_sub_tile<64, 4, 2>(Ark + w, rows, rest, ld, Ark, ld, Ark, ld, w, 1, m0, n0);
 }
 
-int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, int32_t* info, unsigned* flags,
-                         cudaStream_t st) {
+int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, int64_t r, int32_t* info,
+                         unsigned* flags, cudaStream_t st) {
   static TgpPerDeviceOnce attr_once;
   if (tgp_first_use_on_device(attr_once)) {
     constexpr int GSMEM = STAGES * (BM + 64) * BK * 8;
@@ -1335,7 +1319,7 @@ int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, i
         if (Nh[b] <= k) continue;
         const int64_t w = Nh[b] - k < TGP_OB ? Nh[b] - k : TGP_OB, ndiag = tgp_cdiv(w, NB);
         if (j >= ndiag) continue;
-        const int64_t c = (ndiag - j) + tgp_cdiv(Nh[b] - k - w + 1, NB);
+        const int64_t c = (ndiag - j) + tgp_cdiv(Nh[b] - k - w + r, NB);
         ctas = c > ctas ? c : ctas;
       }
       panel_left_batch_kernel<<<dim3((unsigned)B, (unsigned)ctas), PL_THREADS, PL_SMEM, st>>>(pr, k, j, info, flags,
@@ -1345,7 +1329,7 @@ int tgp_batch_potrf_rows(const TgpBatchProb* pr, const int64_t* Nh, int32_t B, i
     const int64_t rest = nmax - k - wmax;   // the largest trailing update belongs to the largest problem
     if (rest > 0) {
       const int tiles_n = (int)tgp_cdiv(rest, 64);
-      const int64_t tiles = tgp_cdiv(rest + 1, BM) * tiles_n;
+      const int64_t tiles = tgp_cdiv(rest + r, BM) * tiles_n;
       gemm_trail_batch_kernel<<<dim3((unsigned)B, (unsigned)tiles), GEMM_THREADS, STAGES * (BM + 64) * BK * 8, st>>>(
           pr, k, tiles_n);
       TGP_LAUNCH_CHECK();
@@ -1371,9 +1355,27 @@ loglike_batch_finish_kernel(const TgpBatchProb* __restrict__ pr, int want_alpha,
   if (threadIdx.x == 0) loglike_finish_body(tmp, p.N, info + blockIdx.x, out + 3 * (int64_t)blockIdx.x);
 }
 
-int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int want_alpha, const int32_t* info, double* out,
-                             cudaStream_t st) {
-  loglike_batch_finish_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, want_alpha, info, out);
+// Several outputs: one CTA per problem with the body of loglike_multi_finish_kernel; alpha (N x r, row-major) holds
+// what the single call's rows hold.
+__global__ void __launch_bounds__(1024)
+loglike_multi_batch_finish_kernel(const TgpBatchProb* __restrict__ pr, int want_alpha,
+                                  const int32_t* __restrict__ info_all, double* __restrict__ out_all) {
+  const TgpBatchProb& p = pr[blockIdx.x];
+  const double* __restrict__ L = p.A;
+  const int64_t N = p.N, ld = p.ld;
+  const double* __restrict__ Y = p.y;
+  const int r = (int)p.r;
+  const double* __restrict__ W = p.alpha;
+  const int64_t wcol = 1, wrow = r;   // output c in column c of alpha
+  const int32_t* __restrict__ info = info_all + blockIdx.x;
+  double* __restrict__ out = out_all + 3 * (int64_t)blockIdx.x;
+#include "multi_finish_body.cuh"
+}
+
+int tgp_batch_loglike_finish(const TgpBatchProb* pr, int32_t B, int64_t r, int want_alpha, const int32_t* info,
+                             double* out, cudaStream_t st) {
+  if (r == 1) loglike_batch_finish_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, want_alpha, info, out);
+  else loglike_multi_batch_finish_kernel<<<(unsigned)B, 1024, 0, st>>>(pr, want_alpha, info, out);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

@@ -17,8 +17,8 @@ constexpr int PM_TILE = 1024;     // training points per shared-memory tile
 // Several outputs (P = MultiOut<..., R>): alpha and mean are row-major (N, r) and (M, r); each thread keeps R pairs of
 // accumulators, evaluates every pair's profile once and applies it to all columns -- each column in the order of the
 // single-output kernel.  The tile shrinks with R so that the staged alpha stays at 16 KB.
-// BATCH (tgp_predict_mean_batch): grid (problems of one profile class, test-point blocks of the largest of them); the
-// problem's slices and descriptor replace the arguments, and every CTA sums all training tiles of its problem in order
+// BATCH (tgp_predict_mean_batch[_multi]): grid (problems of one profile class, test-point blocks of the largest of
+// them); the problem's slices, descriptor and output count replace the arguments, and every CTA sums all training tiles of its problem in order
 // (one split): the single call's sum whenever that call runs unsplit, independent of the other problems.
 template <class P, bool BATCH = false>
 __global__ void __launch_bounds__(PM_THREADS)
@@ -37,7 +37,8 @@ predict_mean_kernel(const double* __restrict__ Xs, int64_t M, const double* __re
     N = pr[b].N;
     alpha = pr[b].alpha;
     mean = pr[b].mean;
-    prof = tgp_batch_profile<P>(kd[b]);
+    if constexpr (OutputsOf<P>::kR > 1) prof = P{tgp_batch_profile<typename OutputsOf<P>::Base>(kd[b]), (int)pr[b].r};
+    else prof = tgp_batch_profile<P>(kd[b]);
     bx = blockIdx.y;
     by = 0;
     nsplit = 1;
@@ -171,19 +172,44 @@ extern "C" int tgp_predict_mean_sum(const double* Xs, int64_t M, const double* X
   return predict_mean_launch(Xs, M, X, N, SumProfile{make_ksumdesc(k)}, alpha, mean, stream);
 }
 
+// P: the policy of profile class cls for the problems' r outputs (one output, or MultiOut padded as mean_multi_launch
+// pads it)
+template <template <class> class Outs>
+static void predict_mean_batch_launch(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int cls,
+                                      dim3 grid, cudaStream_t st) {
+  const double* phi = tgp_phi_device();
+  if (cls == TGP_BATCH_SUM) {
+    using P = typename Outs<SumProfile>::type;
+    predict_mean_kernel<P, true><<<grid, PM_THREADS, 0, st>>>(nullptr, 0, nullptr, 0, P{}, nullptr, nullptr, phi, pr,
+                                                              kd, list);
+  } else {
+    TGP_FAMILY_SWITCH(cls, (predict_mean_kernel<typename Outs<FamilyProfile<FAM>>::type, true>
+                            <<<grid, PM_THREADS, 0, st>>>(nullptr, 0, nullptr, 0,
+                                                          typename Outs<FamilyProfile<FAM>>::type{}, nullptr, nullptr,
+                                                          phi, pr, kd, list)));
+  }
+}
+template <class Q>
+struct OneOut {
+  using type = Q;
+};
+template <int R>
+struct MultiOuts {
+  template <class Q>
+  struct of {
+    using type = MultiOut<Q, R>;
+  };
+};
+
 int tgp_batch_predict_mean(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
-                           int64_t max_m, cudaStream_t st) {
+                           int64_t max_m, int r, cudaStream_t st) {
   const int64_t gy = tgp_cdiv(max_m, PM_THREADS);
   TGP_CHECK_ARG(gy <= 65535, "too many test points in one problem (at most 65535 * 256)");
   const dim3 grid((unsigned)count, (unsigned)gy);
-  const double* phi = tgp_phi_device();
-  if (cls == TGP_BATCH_SUM) {
-    predict_mean_kernel<SumProfile, true><<<grid, PM_THREADS, 0, st>>>(nullptr, 0, nullptr, 0, SumProfile{}, nullptr,
-                                                                      nullptr, phi, pr, kd, list);
-  } else {
-    TGP_FAMILY_SWITCH(cls, (predict_mean_kernel<FamilyProfile<FAM>, true><<<grid, PM_THREADS, 0, st>>>(
-                               nullptr, 0, nullptr, 0, FamilyProfile<FAM>{}, nullptr, nullptr, phi, pr, kd, list)));
-  }
+  if (r == 1) predict_mean_batch_launch<OneOut>(pr, kd, list, cls, grid, st);
+  else if (r <= 2) predict_mean_batch_launch<MultiOuts<2>::of>(pr, kd, list, cls, grid, st);
+  else if (r <= 4) predict_mean_batch_launch<MultiOuts<4>::of>(pr, kd, list, cls, grid, st);
+  else predict_mean_batch_launch<MultiOuts<8>::of>(pr, kd, list, cls, grid, st);
   TGP_LAUNCH_CHECK();
   return TGP_OK;
 }

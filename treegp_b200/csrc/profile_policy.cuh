@@ -37,7 +37,8 @@ static inline KSumDesc make_ksumdesc(const tgp_kernel_sum* ks) {
 }
 
 // Several outputs sharing one kernel: the policy P with nrhs = r columns of alpha (row-major (N, r)), padded to R
-// columns where a kernel keeps them in registers or shared memory.  OutputsOf<P>::kR is 1 for a plain policy.
+// columns where a kernel keeps them in registers or shared memory.  OutputsOf<P>::kR is 1 for a plain policy, and
+// OutputsOf<P>::Base the policy of one output.
 template <class P, int R>
 struct MultiOut : P {
   int nrhs;
@@ -45,10 +46,12 @@ struct MultiOut : P {
 template <class P>
 struct OutputsOf {
   static constexpr int kR = 1;
+  using Base = P;
 };
 template <class P, int R>
 struct OutputsOf<MultiOut<P, R>> {
   static constexpr int kR = R;
+  using Base = P;
 };
 
 #ifdef __CUDACC__

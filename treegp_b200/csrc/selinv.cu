@@ -481,7 +481,8 @@ int tgp_batch_selinv(const TgpBatchProb* pr, double* const* scr, const TgpBatchP
 
 // grid: (tile, term, problem of the list); the single call's contraction on each problem, Z in its workspace block and
 // the tile partials at the front of its scratch.  The problem's profile is staged in shared memory: the body indexes a
-// sum's terms by blockIdx.y, which a copy in registers could only do from the stack.
+// sum's terms by blockIdx.y, which a copy in registers could only do from the stack.  P = MultiOut<...>: the problem's
+// r outputs (alpha N x r), as tgp_loglike_grad_multi contracts them.
 template <class P>
 __global__ void __launch_bounds__(GT_THREADS)
 grad_contract_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* __restrict__ descs,
@@ -491,12 +492,16 @@ grad_contract_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* 
   const int64_t N = pr[b].N, nt = (N + GT - 1) / GT;
   if ((int64_t)blockIdx.x >= nt * (nt + 1) / 2) return;
   if (P::kSum && (int)blockIdx.y >= descs[b].nterms) return;
-  __shared__ P prof_s;   // P holds one descriptor: the sum's, or a family's single term
-  static_assert(sizeof(prof_s.desc) == sizeof(P) && sizeof(P) % 4 == 0, "a profile is its descriptor");
+  __shared__ P prof_s;   // P holds one descriptor (the sum's, or a family's single term), and for r outputs nrhs
+  static_assert((sizeof(prof_s.desc) == sizeof(P) || OutputsOf<P>::kR > 1) && sizeof(prof_s.desc) % 4 == 0,
+                "a profile is its descriptor");
   {
     const int* src = reinterpret_cast<const int*>(P::kSum ? (const void*)&descs[b] : (const void*)&descs[b].term[0]);
-    int* dst = reinterpret_cast<int*>(&prof_s);
-    for (int i = threadIdx.x; i < (int)(sizeof(P) / 4); i += GT_THREADS) dst[i] = src[i];
+    int* dst = reinterpret_cast<int*>(&prof_s.desc);
+    for (int i = threadIdx.x; i < (int)(sizeof(prof_s.desc) / 4); i += GT_THREADS) dst[i] = src[i];
+    if constexpr (OutputsOf<P>::kR > 1) {
+      if (threadIdx.x == 0) prof_s.nrhs = (int)pr[b].r;
+    }
   }
   __syncthreads();
   const P& prof = prof_s;
@@ -509,18 +514,24 @@ grad_contract_batch_kernel(const TgpBatchProb* __restrict__ pr, const KSumDesc* 
 #include "grad_contract_body.cuh"
 }
 
+template <class Q>
+static void grad_contract_batch_launch(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list,
+                                       double* const* scr, int r, dim3 grid, cudaStream_t st) {
+  const double* phi = tgp_phi_device();
+  if (r == 1) grad_contract_batch_kernel<Q><<<grid, GT_THREADS, 0, st>>>(pr, kd, list, scr, phi);
+  else grad_contract_batch_kernel<MultiOut<Q, TGP_MAX_RHS>><<<grid, GT_THREADS, 0, st>>>(pr, kd, list, scr, phi);
+}
+
 int tgp_batch_grad_contract(const TgpBatchProb* pr, const KSumDesc* kd, const int32_t* list, int32_t count, int cls,
-                            double* const* scr, int64_t max_n, int max_terms, cudaStream_t st) {
+                            double* const* scr, int64_t max_n, int max_terms, int r, cudaStream_t st) {
   const int64_t ntiles = grad_tiles(max_n);
   TGP_CHECK_ARG(ntiles < (1ll << 31), "matrix too large for one launch");
-  const double* phi = tgp_phi_device();
   for (int32_t z0 = 0; z0 < count; z0 += 65535) {   // gridDim.z <= 65535
     const dim3 grid((unsigned)ntiles, (unsigned)max_terms, (unsigned)std::min(count - z0, 65535));
     if (cls == TGP_BATCH_SUM) {
-      grad_contract_batch_kernel<SumProfile><<<grid, GT_THREADS, 0, st>>>(pr, kd, list + z0, scr, phi);
+      grad_contract_batch_launch<SumProfile>(pr, kd, list + z0, scr, r, grid, st);
     } else {
-      TGP_FAMILY_SWITCH(cls, (grad_contract_batch_kernel<FamilyProfile<FAM>><<<grid, GT_THREADS, 0, st>>>(
-                                 pr, kd, list + z0, scr, phi)));
+      TGP_FAMILY_SWITCH(cls, (grad_contract_batch_launch<FamilyProfile<FAM>>(pr, kd, list + z0, scr, r, grid, st)));
     }
     TGP_LAUNCH_CHECK();
   }

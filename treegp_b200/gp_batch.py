@@ -17,6 +17,7 @@ import torch
 from scipy import optimize
 
 from . import _cabi, backend
+from .gp_interp import TWO_PCF_NEEDS_1D_Y
 from .kernels import descriptor_params, eval_kernel, lower, lower_jacobian
 from .log_likelihood import log_likelihood
 from .two_pcf import two_pcf
@@ -93,7 +94,9 @@ def lockstep_minimize(evaluate, x0s, jac=False):
 
 
 class GPInterpolationBatch(object):
-    """B independent Gaussian-process interpolations of scalar surfaces, put through the device together.
+    """B independent Gaussian-process interpolations, put through the device together.  Each problem has one scalar
+    field, or r fields (1 <= r <= TGP_MAX_RHS, the same r for all problems) that share its kernel, as a 2-D y does
+    in ``GPInterpolation``.
 
     Constructor keywords mean what they mean in ``GPInterpolation``:
 
@@ -128,9 +131,10 @@ class GPInterpolationBatch(object):
         self._solved = None
 
     def initialize(self, Xs, ys, y_errs=None):
-        """Attach B problems: lists of positions (N_b, ndim), values (N_b,) and optional errors (N_b,).  Per problem
+        """Attach B problems: lists of positions (N_b, ndim), values (N_b,) -- or (N_b, r) for r outputs sharing the
+        problem's kernel, one r for every problem -- and optional errors (N_b,), shared by the outputs.  Per problem
         what GPInterpolation.initialize does: a fresh copy of the kernel, zero errors when none are given, the white
-        noise added in quadrature and the normalising mean."""
+        noise added in quadrature and the normalising mean (one per output)."""
         B = len(Xs)
         if B == 0 or len(ys) != B or (y_errs is not None and len(y_errs) != B):
             raise ValueError("Xs, ys and y_errs must be lists of the same, non-zero length (%d, %d, %s)"
@@ -139,14 +143,20 @@ class GPInterpolationBatch(object):
         if len(templates) != B:
             raise ValueError("%d kernel strings for %d problems" % (len(templates), B))
         ndims = set()
+        shape0 = np.shape(ys[0])
         for b in range(B):
             X, y = np.asarray(Xs[b]), np.asarray(ys[b])
-            if y.ndim != 1:
-                raise ValueError("problem %d: y must be 1-D (one output per problem); got shape %r" % (b, y.shape))
+            if y.ndim not in (1, 2) or y.ndim != len(shape0):
+                raise ValueError("problem %d: y has shape %r; a batch takes 1-D ys (N_b,) or 2-D ys (N_b, r), the same "
+                                 "for all problems (problem 0: %r)" % (b, y.shape, shape0))
+            if y.ndim == 2 and not (1 <= y.shape[1] <= _cabi.MAX_RHS and y.shape[1] == shape0[1]):
+                raise ValueError("problem %d: y has %d outputs; a batch takes one r, 1 <= r <= %d (TGP_MAX_RHS), for "
+                                 "all problems (problem 0: %d)" % (b, y.shape[1], _cabi.MAX_RHS, shape0[1]))
             if X.ndim != 2 or X.shape[0] != len(y) or len(y) == 0:
                 raise ValueError("problem %d: X must have shape (N, ndim) with N = len(y) >= 1; got %r" % (b, X.shape))
-            if y_errs is not None and y_errs[b] is not None and np.shape(y_errs[b]) != y.shape:
-                raise ValueError("problem %d: y_err must have the shape of y" % b)
+            if y_errs is not None and y_errs[b] is not None and np.shape(y_errs[b]) != (len(y),):
+                raise ValueError("problem %d: y_err must have shape (N,) = (%d,), shared by the outputs; got %r"
+                                 % (b, len(y), np.shape(y_errs[b])))
             if len(y) > _cabi.BATCH_MAX_N:
                 raise ValueError("problem %d has %d points; a batch takes at most %d per problem (TGP_BATCH_MAX_N) -- "
                                  "use GPInterpolation for it" % (b, len(y), _cabi.BATCH_MAX_N))
@@ -157,14 +167,21 @@ class GPInterpolationBatch(object):
         self._X, self._y, self._y_err, self._mean, self._spatial_average = [], [], [], [], []
         for b in range(B):
             y = ys[b]
-            y_err = np.zeros_like(y) if y_errs is None or y_errs[b] is None else y_errs[b]
+            multi = np.ndim(y) == 2
+            y_err = (np.zeros(len(y)) if multi else np.zeros_like(y)) if y_errs is None or y_errs[b] is None else y_errs[b]
             self._X.append(Xs[b])
             self._y.append(y)
-            self._spatial_average.append(np.zeros(len(Xs[b][:, 0])))
+            self._spatial_average.append(np.zeros(np.shape(y)))
             if self.white_noise > 0:
                 y_err = np.sqrt(np.array(y_err, dtype=float) ** 2 + self.white_noise ** 2)
             self._y_err.append(y_err)
-            self._mean.append(np.mean(y - self._spatial_average[b]) if self.normalize else 0.0)
+            if not self.normalize:
+                self._mean.append(0.0)
+            elif multi:   # column by column, as GPInterpolation.initialize: each output's mean as on its own
+                res = np.asarray(y - self._spatial_average[b])
+                self._mean.append(np.array([np.mean(np.ascontiguousarray(res[:, c])) for c in range(res.shape[1])]))
+            else:
+                self._mean.append(np.mean(y - self._spatial_average[b]))
         self._dev = None
         self._solved = None
 
@@ -175,7 +192,7 @@ class GPInterpolationBatch(object):
         """Concatenated X, residual y and y_err^2 of all problems on the device (built once per initialize)."""
         if self._dev is None:
             X = torch.cat([backend.as_points(X) for X in self._X])
-            y = backend.to_device(np.concatenate([np.asarray(self._residual(b), dtype=np.float64).reshape(-1)
+            y = backend.to_device(np.concatenate([np.asarray(self._residual(b), dtype=np.float64)
                                                   for b in range(len(self._X))]))
             e2 = backend.to_device(np.concatenate([np.asarray(e, dtype=np.float64).reshape(-1) ** 2
                                                    for e in self._y_err]))
@@ -234,6 +251,8 @@ class GPInterpolationBatch(object):
         switch GPInterpolation honours), the "log-likelihood" searches use the analytic gradient: one batched
         value-and-gradient call per round."""
         B = len(self._X)
+        if np.ndim(self._y[0]) == 2 and self.optimizer in ["two-pcf", "anisotropic"]:
+            raise ValueError(TWO_PCF_NEEDS_1D_Y)
         self._init_theta = [copy.deepcopy(k).theta for k in self.kernels]
         self._solved = None
         if self.optimizer == "log-likelihood" and log_likelihood.ANALYTIC_GRADIENT:
@@ -298,7 +317,8 @@ class GPInterpolationBatch(object):
                 raise ValueError("problem %d: positions must have shape (M, %d); got %r" % (b, ndim, np.shape(x)))
 
     def predict(self, Xs_new, return_cov=False):
-        """Posterior means at the positions Xs_new[b] (M_b, ndim) of every problem: a list of B arrays."""
+        """Posterior means at the positions Xs_new[b] (M_b, ndim) of every problem: a list of B arrays, (M_b,), or
+        (M_b, r) for r outputs."""
         if return_cov:
             raise ValueError("GPInterpolationBatch predicts means only; use GPInterpolation for a covariance")
         if len(Xs_new) != len(self._X):
@@ -309,21 +329,24 @@ class GPInterpolationBatch(object):
         Xs = torch.cat([backend.as_points(x) for x in Xs_new])
         mean = backend.predict_mean_batch(Xs, ssizes, X, sizes, descs, alpha).cpu().numpy()
         soff = backend.batch_offsets(ssizes)
-        return [mean[soff[b]:soff[b + 1]] + self._mean[b] + np.zeros(ssizes[b]) for b in range(len(sizes))]
+        return [mean[soff[b]:soff[b + 1]] + self._mean[b] + np.zeros((ssizes[b],) + mean.shape[1:])
+                for b in range(len(sizes))]
 
     def predict_var(self, Xs_new):
         """Posterior means and DIAGONAL predictive variances at the positions Xs_new[b] (M_b, ndim) of every problem:
         (means, vars), two lists of B arrays.  The means are predict's; the variances are what
         GPInterpolation.predict_var returns for the problem, bit for bit with its dense solve (residual space: the
         normalising mean does not enter).  All problems' test points go through one batched call
-        (tgp_predict_var_batch), which factorises into a workspace of its own."""
+        (tgp_predict_var_batch), which factorises into a workspace of its own.  With r outputs the means are (M_b, r)
+        and the variances (M_b,), shared by the outputs: they do not depend on y, so one output is factorised."""
         self._check_positions(Xs_new)
         means = self.predict(Xs_new)
         descs, _ = self._ensure_solved()
         X, y, e2, sizes, _ = self._device_data()
         ssizes = [len(m) for m in means]
         Xs = torch.cat([backend.as_points(x) for x in Xs_new])
-        var, info = backend.predict_var_batch(Xs, ssizes, X, y, e2, sizes, descs, budget_bytes=self.WORK_BUDGET)
+        y1 = y if y.dim() == 1 else y[:, 0].contiguous()
+        var, info = backend.predict_var_batch(Xs, ssizes, X, y1, e2, sizes, descs, budget_bytes=self.WORK_BUDGET)
         self._raise_on_info(info, "tgp_loglike_batch")
         var = var.cpu().numpy()
         soff = backend.batch_offsets(ssizes)
@@ -333,7 +356,8 @@ class GPInterpolationBatch(object):
         """Leave-one-out predictions at every training point of every problem, without refitting: (means, vars), two
         lists of B arrays in each problem's own order, as GPInterpolation.loo_predict gives them -- mean_i = y_i -
         alpha_i / Z_ii plus the normalising mean, var_i = 1 / Z_ii - y_err_i^2, Z = (K + diag(y_err^2))^-1.  One
-        batched call (tgp_loo_batch) factorises and inverts every problem in a workspace of its own."""
+        batched call (tgp_loo_batch) factorises and inverts every problem in a workspace of its own.  With r outputs
+        the means are (N_b, r), mean_ic = y_ic - alpha_ic / Z_ii, and the variances (N_b,)."""
         descs = self._descriptors()
         X, y, e2, sizes, off = self._device_data()
         mean, var, info = backend.loo_batch(X, y, e2, sizes, descs, budget_bytes=self.WORK_BUDGET)
@@ -344,7 +368,7 @@ class GPInterpolationBatch(object):
 
     def return_log_likelihood(self, thetas=None):
         """Marginal log-likelihood of every problem for its current kernel, or for thetas[b] if given: an array of B
-        values from one batched call."""
+        values from one batched call (with r outputs the joint value, the sum over the outputs)."""
         kernels = [copy.deepcopy(k) for k in self.kernels]
         if thetas is not None:
             kernels = [k.clone_with_theta(t) for k, t in zip(kernels, thetas)]

@@ -317,8 +317,7 @@ class GPInterpolation(object):
     def _check_2pcf_output(self, always=False):
         """The 2-point correlation function fit is defined for one scalar field."""
         if np.ndim(self._y) == 2 and (always or self.optimizer in ["two-pcf", "anisotropic"]):
-            raise ValueError("the two-pcf / anisotropic fit and return_2pcf need a 1-D y; with several outputs use "
-                             "optimizer='log-likelihood' or 'none'")
+            raise ValueError(TWO_PCF_NEEDS_1D_Y)
 
     def return_log_likelihood(self, theta=None):
         """Marginal log-likelihood of the current data for the current kernel, or for `theta` if given
@@ -366,6 +365,11 @@ class GPInterpolation(object):
                 plt.ylabel(r"$\Delta y$", fontsize=16)
             plt.title(title, fontsize=16)
         return fig
+
+
+# the 2-point correlation function fit is defined for one scalar field (GPInterpolation and GPInterpolationBatch)
+TWO_PCF_NEEDS_1D_Y = ("the two-pcf / anisotropic fit and return_2pcf need a 1-D y; with several outputs use "
+                      "optimizer='log-likelihood' or 'none'")
 
 
 def _unsort(t, order):
